@@ -24,6 +24,11 @@ over BASELINE.json configs[1] (C2): 10 000 files x 100 000 regions = 1e9 query i
 `--scaling weak` (default): every rank owns `--files` files (1e9 queries per GPU); `--scaling strong`: `--files` files in
 total.  `--impl reference` times the oracle with all host threads instead (rank 0 only).  Multi-GPU (torchrun): files
 are sharded across ranks (rank r owns files [r*F, (r+1)*F)), universe replicated, no collective on the C2 data path.
+
+`--dump-outputs DIR` writes rank 0's C2 result of the last timed step as float64 .npy files: token_ids.npy and
+file_token_offsets.npy (raw per-file offsets into the ids, before the per-file [unk] rule).  An array longer than
+DUMP_MAX_VALUES is written as a fixed, seeded sample, with the sampled positions in <name>_positions.npy.  The inputs are
+counter-based (gtars_b200/synth.py), so the same arguments give the same files on every run and every build.
 """
 from __future__ import annotations
 
@@ -69,7 +74,13 @@ def parse_args():
     ap.add_argument("--sub-scale", type=float, default=1.0, help="scale factor on the sizes of the c3/c4/c5 sub-records")
     ap.add_argument("--parity-files", type=int, default=1000, help="files of the full-size C2 result checked against the oracle")
     ap.add_argument("--no-pcie-probe", action="store_true")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write rank 0's result of the last timed step (token ids and per-file "
+                                                          "token offsets) to DIR/<name>.npy as float64, for output-by-output "
+                                                          "comparison of two builds")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    return args
 
 
 def workload_config(args, world):
@@ -204,6 +215,27 @@ def run_reference(args, rank, world):
         "e2e": {"value": value, "unit": UNIT, "h2d_bytes_per_step": 0, "d2h_bytes_per_step": 0},
         "gpu_launches": 0,
     }))
+
+
+# --dump-outputs: an array longer than this is dumped as a fixed, seeded sample of its positions, and the sorted positions
+# are dumped beside it; ids + positions + offsets + positions stay under 64 MB of float64 (exact for u32 ids and offsets < 2^53).
+DUMP_MAX_VALUES = 1 << 20
+
+
+def dump_positions(n: int, seed: int):
+    """None when all n values fit the dump, else DUMP_MAX_VALUES distinct sorted positions of [0, n), the same on every run."""
+    if n <= DUMP_MAX_VALUES:
+        return None
+    return np.sort(np.random.default_rng(seed).choice(n, DUMP_MAX_VALUES, replace=False))
+
+
+def write_dump(out_dir: str, arrays: dict):
+    """arrays: name -> (values, positions or None); everything is written as float64."""
+    os.makedirs(out_dir, exist_ok=True)
+    for name, (values, pos) in arrays.items():
+        np.save(os.path.join(out_dir, f"{name}.npy"), np.asarray(values).astype(np.float64))
+        if pos is not None:
+            np.save(os.path.join(out_dir, f"{name}_positions.npy"), pos.astype(np.float64))
 
 
 def digest64(*arrays) -> str:
@@ -786,6 +818,12 @@ def main():
         hits = int(d_total.item())
         assert hits <= cap, "output capacity too small for the synthetic workload"
         n_empty_files = int((d_file_tok[1:] == d_file_tok[:-1]).sum().item())
+        dump = None
+        if args.dump_outputs and rank == 0:
+            # what a caller of this path receives: the ids of all files and each file's offset into them
+            dump = {name: (t, dump_positions(len(t), seed)) for seed, (name, t) in
+                    enumerate((("token_ids", d_ids[:hits]), ("file_token_offsets", d_file_tok)))}
+            dump_index = {name: torch.from_numpy(pos).to(dev) for name, (_, pos) in dump.items() if pos is not None}
 
         # ---- timed region: K back-to-back steps, CUDA events on the launching stream ---------------------------------
         sampler = ClockSampler(local_rank)
@@ -801,6 +839,8 @@ def main():
         ev1.record(stream)
         stream.synchronize()
         torch.cuda.synchronize()
+        if dump is not None:  # copied before the untimed steps below rewrite the same buffers
+            dump = {name: (t[dump_index[name]] if pos is not None else t.clone(), pos) for name, (t, pos) in dump.items()}
         D.barrier()
         kernel_ms = ctx.timing_read()
         ctx.timing_enable(False)
@@ -815,6 +855,10 @@ def main():
         clocks = sampler.stop()
         clocks["window"] = "timed region + 0.5 s of the identical steps right behind it"
         ms_per_step = D.max(ev0.elapsed_time(ev1) / args.steps)
+        if dump is not None:
+            write_dump(args.dump_outputs, {name: (t.cpu().numpy().view(np.uint32) if t.dtype == torch.int32 else t.cpu().numpy(), pos)
+                                           for name, (t, pos) in dump.items()})
+            del dump, dump_index
 
     total_queries = D.sum(float(n))
     value = total_queries / (ms_per_step * 1e-3)

@@ -65,6 +65,28 @@ def test_digest_is_order_sensitive():
     assert b.digest64(a[:5], a[5:]) == b.digest64(a)
 
 
+def test_dump_outputs_sample_is_fixed_bounded_and_float64(tmp_path):
+    b = _bench()
+    assert b.dump_positions(b.DUMP_MAX_VALUES, 0) is None
+    n = 1_000_000_000
+    p = b.dump_positions(n, 0)
+    assert len(p) == b.DUMP_MAX_VALUES and np.all(np.diff(p) > 0) and p[0] >= 0 and p[-1] < n
+    assert np.array_equal(p, b.dump_positions(n, 0)) and not np.array_equal(p, b.dump_positions(n, 1))
+    ids = np.array([0, 7, 0xFFFFFFFF], dtype=np.uint32)
+    b.write_dump(str(tmp_path / "d"), {"ids": (ids, None), "offs": (np.arange(5, dtype=np.int64), np.array([0, 2, 9]))})
+    got = {f: np.load(tmp_path / "d" / f) for f in sorted(os.listdir(tmp_path / "d"))}
+    assert sorted(got) == ["ids.npy", "offs.npy", "offs_positions.npy"] and all(a.dtype == np.float64 for a in got.values())
+    assert got["ids.npy"].tolist() == [0, 7, 0xFFFFFFFF] and got["offs_positions.npy"].tolist() == [0, 2, 9]
+    # four arrays at the cap (ids, offsets and their positions) stay within 64 MB
+    assert 4 * (8 * b.DUMP_MAX_VALUES + 128) <= 64 << 20
+
+
+def test_steps_must_be_positive():
+    r = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--impl", "reference", "--steps", "0"],
+                       capture_output=True, text=True, timeout=120, cwd=ROOT)
+    assert r.returncode == 2 and "--steps" in r.stderr
+
+
 def test_marshal_compact_matches_numpy():
     """gtgpu_marshal_compact is host code: runs cut at chromosome changes and file boundaries, u16 widths, exceptions."""
     from gtars_b200 import ffi
