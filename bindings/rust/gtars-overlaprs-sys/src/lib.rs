@@ -100,6 +100,19 @@ extern "C" {
     pub fn gtgpu_score_barcodes(index: *mut gtgpu_index, n: u64, chr: *const u32, start: *const u32, end: *const u32,
                                 barcode_id: *const u32, n_barcodes: u32, out_barcode_offsets: *mut u64,
                                 out_peaks: *mut *mut gtgpu_buf, out_counts: *mut *mut gtgpu_buf) -> i32;
+    pub fn gtgpu_score_matrix_text(index: *mut gtgpu_index, text: *const u8, n_bytes: u64, n_names: u32, names: *const u8,
+                                   name_offsets: *const u32, mode: i32, n_cols: u64, out_row: *mut u32) -> i32;
+    pub fn gtgpu_score_matrix_gz(index: *mut gtgpu_index, n_members: u64, gz: *const u8, member_offsets: *const u64, n_names: u32,
+                                 names: *const u8, name_offsets: *const u32, mode: i32, n_cols: u64, out_row: *mut u32) -> i32;
+    pub fn gtgpu_score_barcodes_text(index: *mut gtgpu_index, text: *const u8, n_bytes: u64, n_names: u32, names: *const u8,
+                                     name_offsets: *const u32, out_n_barcodes: *mut u32, out_barcode_names: *mut *mut gtgpu_buf,
+                                     out_barcode_name_offsets: *mut *mut gtgpu_buf, out_barcode_offsets: *mut *mut gtgpu_buf,
+                                     out_peaks: *mut *mut gtgpu_buf, out_counts: *mut *mut gtgpu_buf) -> i32;
+    pub fn gtgpu_score_barcodes_gz(index: *mut gtgpu_index, n_members: u64, gz: *const u8, member_offsets: *const u64, n_names: u32,
+                                   names: *const u8, name_offsets: *const u32, out_n_barcodes: *mut u32,
+                                   out_barcode_names: *mut *mut gtgpu_buf, out_barcode_name_offsets: *mut *mut gtgpu_buf,
+                                   out_barcode_offsets: *mut *mut gtgpu_buf, out_peaks: *mut *mut gtgpu_buf,
+                                   out_counts: *mut *mut gtgpu_buf) -> i32;
     pub fn gtgpu_igd_build(ctx: *mut gtgpu_ctx, n_files: u64, file_offsets: *const u64, n_chroms: u32, chr: *const u32,
                            start: *const u32, end: *const u32, out_igd: *mut *mut gtgpu_igd) -> i32;
     pub fn gtgpu_igd_free(igd: *mut gtgpu_igd) -> i32;

@@ -50,6 +50,7 @@ def lib():
             "gth_irs_any": (C.c_int, [vp, vp, i32, vp]),
             "gth_consensus_new": (vp, [vp, cp]), "gth_consensus_free": (None, [vp]), "gth_consensus_len": (u64, [vp]),
             "gth_region_scoring": (C.c_int, [vp, u64, vp, C.c_int, vp]), "gth_barcode_scoring": (vp, [vp, cp]),
+            "gth_region_scoring_device": (C.c_int, [vp, u64, vp, C.c_int, vp]), "gth_barcode_scoring_device": (vp, [vp, cp]),
             "gth_tokenizer_new": (vp, [vp, cp, C.c_int]), "gth_tokenizer_free": (None, [vp]),
             "gth_tokenizer_vocab_size": (u64, [vp]), "gth_tokenizer_token_to_id": (i64, [vp, cp]),
             "gth_tokenizer_id_to_token": (cp, [vp, u32]), "gth_tokenizer_special": (cp, [vp, C.c_int]),
@@ -318,19 +319,23 @@ class ConsensusSet:
         return int(lib().gth_consensus_len(self._h))
 
 
-def region_scoring_from_fragments(fragment_files, consensus, mode=SCORING_ATAC):
-    """gtars_scoring::region_scoring_from_fragments: uint32 [n_files, len(consensus)] (files in the given order)."""
+def region_scoring_from_fragments(fragment_files, consensus, mode=SCORING_ATAC, device_parse: bool = False):
+    """gtars_scoring::region_scoring_from_fragments: uint32 [n_files, len(consensus)] (files in the given order).
+    device_parse=True parses every file's text on the device (gtgpu_score_matrix_text / _gz), any file size."""
     files = [os.fsencode(p) for p in fragment_files]
     arr = (C.c_char_p * max(len(files), 1))(*files)
     out = np.zeros((len(files), len(consensus)), dtype=np.uint32)
-    if lib().gth_region_scoring(consensus._h, len(files), arr, mode, out.ctypes.data):
+    fn = lib().gth_region_scoring_device if device_parse else lib().gth_region_scoring
+    if fn(consensus._h, len(files), arr, mode, out.ctypes.data):
         _fail()
     return out
 
 
-def barcode_scoring_from_fragments(fragment_file, consensus):
-    """gtars_scoring::barcode_scoring_from_fragments: {barcode: {peak index: count}}."""
-    named = _take_lists(lib().gth_barcode_scoring(consensus._h, os.fsencode(fragment_file)), named=True)
+def barcode_scoring_from_fragments(fragment_file, consensus, device_parse: bool = False):
+    """gtars_scoring::barcode_scoring_from_fragments: {barcode: {peak index: count}}, barcodes in first-appearance order.
+    device_parse=True parses the text and numbers the barcodes on the device (gtgpu_score_barcodes_text / _gz)."""
+    fn = lib().gth_barcode_scoring_device if device_parse else lib().gth_barcode_scoring
+    named = _take_lists(fn(consensus._h, os.fsencode(fragment_file)), named=True)
     return {bc: dict(zip(flat[0::2], flat[1::2])) for bc, flat in named}
 
 

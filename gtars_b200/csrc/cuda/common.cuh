@@ -8,6 +8,7 @@
 #include <map>
 #include <mutex>
 #include <string>
+#include <utility>
 #include <vector>
 
 #include "../../../include/gtars_gpu.h"
@@ -233,7 +234,8 @@ enum ScratchRole {
     SC_CHR = 0, SC_START, SC_END, SC_BARCODE, SC_OUT_IDS, SC_OUT_IDS2, SC_OUT_OFFS, SC_FILE_OFFS, SC_FILE_TOK,
     SC_FILE_TOK2, SC_TILE_STATUS, SC_TILE_FILE, SC_MISC, SC_COUNTS, SC_IN2_CHR, SC_IN2_START, SC_IN2_END,
     SC_IN3_CHR, SC_IN3_START, SC_IN3_END, SC_SET_ID, SC_MATRIX, SC_ING_0, SC_ING_1, SC_ING_2, SC_ING_3, SC_ING_4, SC_ING_5,
-    SC_ING_6, SC_ING_7, SC_GZ_IN, SC_GZ_OUT, SC_GZ_MOFF, SC_GZ_OOFF, SC_GZ_STATUS, SC_CNT_KEYS, SC_CNT_RES, SC_CNT_POS, SC_CNT_RUNS, SC_N_ROLES
+    SC_ING_6, SC_ING_7, SC_GZ_IN, SC_GZ_OUT, SC_GZ_MOFF, SC_GZ_OOFF, SC_GZ_STATUS, SC_CNT_KEYS, SC_CNT_RES, SC_CNT_POS, SC_CNT_RUNS,
+    SC_WIN_A, SC_WIN_B, SC_N_ROLES
 };
 
 // kernels.cu
@@ -314,6 +316,58 @@ int32_t radix_group_values(gtgpu_ctx* ctx, uint64_t n_cap, const uint32_t* keys,
                            uint64_t* out_offsets, uint64_t* d_total);
 
 // ingest.cu / inflate.cu (the caller holds ctx->mu)
+struct NameTable {
+    const char* blob;             // names back to back
+    const uint32_t* offsets;      // n_names + 1
+    const unsigned long long* hash;  // FNV-1a of every name, sorted ascending
+    const uint32_t* hash_id;      // name id of the k-th sorted hash
+    uint32_t n_names;
+};
+// the caller's chromosome names -> scratch SC_SET_ID
+int32_t upload_name_table(gtgpu_ctx* ctx, uint32_t n_names, const char* names, const uint32_t* name_offsets, NameTable* out);
+// What the fragment parse checks and carries: tokenize_fragment_file needs fields 1 and 2 as u32 and the barcode;
+// Fragment::from_str (scoring) needs field 4 as well, and the count matrix has no use for the barcode.
+enum FragMode { FRAG_TOKENIZE = 0, FRAG_SCORE_MATRIX = 1, FRAG_SCORE_BARCODES = 2 };
+struct FragParse {
+    uint32_t n_lines = 0;
+    uint32_t bad_line = 0xFFFFFFFFu;  // 0-based index of the first malformed line of the text, or none
+    uint32_t n = 0;                   // fragments (0 when a line was malformed)
+    uint32_t *chr = nullptr, *start = nullptr, *end = nullptr;  // scratch SC_CHR / SC_START / SC_END
+    unsigned long long* h = nullptr;                             // barcode hash, byte offset and length (not for the matrix)
+    uint32_t *bo = nullptr, *bl = nullptr;
+    uint32_t *free0 = nullptr, *free1 = nullptr, *free2 = nullptr;  // line-sized scratch the caller may reuse
+    void* tmp = nullptr;                                           // scan temp for line-sized arrays
+    uint32_t* flags = nullptr;                                     // device words [1..3], zeroed for the caller
+};
+// d_text: 0 < n_bytes < 0xFFFFFFF0 bytes of device text, 16-byte aligned.  Synchronises the ctx stream.
+int32_t parse_fragments_locked(gtgpu_ctx* ctx, const char* d_text, uint64_t n_bytes, const NameTable& nt, FragMode mode,
+                               FragParse* out);
+// A device buffer owned by one call, grown while keeping its first `keep` bytes.
+struct DevMem {
+    void* ptr = nullptr;
+    size_t cap = 0;
+    DevMem() = default;
+    DevMem(const DevMem&) = delete;
+    DevMem& operator=(const DevMem&) = delete;
+    ~DevMem();
+    int32_t reserve(size_t bytes, size_t keep, cudaStream_t st);
+    void swap(DevMem& o) { std::swap(ptr, o.ptr); std::swap(cap, o.cap); }
+    uint32_t* u32() const { return static_cast<uint32_t*>(ptr); }
+};
+// Barcodes of one fragment file over all its windows (scoring): dense ids in first-appearance order, only barcodes seen on a
+// chromosome of the name table kept.  chr / start / end / bc hold every fragment of the file once finish() has run.
+struct FragBarcodeTable {
+    DevMem chr, start, end, fidx, known, hlen, bc;
+    DevMem keys, first, soff, arena;
+    uint64_t n = 0, distinct = 0, cap = 0, used = 0;
+    int32_t add_window(gtgpu_ctx* ctx, const char* d_text, const FragParse& fp, uint32_t n_names);
+    // *out_names: the kept barcodes' bytes back to back (elem_size 1); *out_name_offsets: n_kept + 1 u64 offsets into them
+    int32_t finish(gtgpu_ctx* ctx, uint32_t* n_kept, gtgpu_buf** out_names, gtgpu_buf** out_name_offsets);
+};
+// inflate.cu: H2D of gzip members + inflate; the text stays in scratch SC_GZ_OUT
+int32_t check_members(uint64_t n_members, const uint8_t* gz, const uint64_t* member_offsets, const char* who);
+int32_t gunzip_locked(gtgpu_ctx* ctx, uint64_t n_members, const uint8_t* gz, const uint64_t* member_offsets,
+                      uint64_t* out_member_offsets, uint8_t** d_text, uint64_t* n_text);
 int32_t tokenize_bed_locked(gtgpu_index* ix, const char* text, uint64_t n_bytes, uint32_t n_names, const char* names,
                             const uint32_t* name_offsets, uint32_t unk_id, gtgpu_buf** out_ids);
 int32_t tokenize_fragments_text_locked(gtgpu_index* ix, const char* text, uint64_t n_bytes, uint32_t n_names, const char* names,

@@ -576,7 +576,7 @@ namespace gtgpu {
 
 // H2D of the members + inflate; the text stays on the device in scratch SC_GZ_OUT (*d_text, *n_text bytes, 64 bytes of
 // padding behind it).  The caller holds ctx->mu.  out_member_offsets (host, n_members + 1) may be null.
-static int32_t gunzip_locked(gtgpu_ctx* ctx, uint64_t n_members, const uint8_t* gz, const uint64_t* member_offsets,
+int32_t gunzip_locked(gtgpu_ctx* ctx, uint64_t n_members, const uint8_t* gz, const uint64_t* member_offsets,
                              uint64_t* out_member_offsets, uint8_t** d_text, uint64_t* n_text) {
     // output size of every member from its trailer (ISIZE, RFC 1952): the text of a member must be < 4 GiB
     std::vector<uint64_t> oo(n_members + 1, 0), rebased(n_members + 1, 0);
@@ -612,7 +612,7 @@ static int32_t gunzip_locked(gtgpu_ctx* ctx, uint64_t n_members, const uint8_t* 
     return gunzip_device(ctx, n_members, d_gz, d_mo, d_oo, d_out, d_status, h_status);
 }
 
-static int32_t check_members(uint64_t n_members, const uint8_t* gz, const uint64_t* member_offsets, const char* who) {
+int32_t check_members(uint64_t n_members, const uint8_t* gz, const uint64_t* member_offsets, const char* who) {
     if (n_members && (!gz || !member_offsets)) return fail(GTGPU_ERR_INVALID, std::string(who) + ": null argument");
     for (uint64_t k = 0; k < n_members; ++k)
         if (member_offsets[k] > member_offsets[k + 1]) return fail(GTGPU_ERR_INVALID, std::string(who) + ": member_offsets not monotone");

@@ -62,14 +62,6 @@ __global__ void ingest_newline_positions_kernel(uint64_t n_bytes, const char* __
     }
 }
 
-struct NameTable {
-    const char* blob;             // names back to back
-    const uint32_t* offsets;      // n_names + 1
-    const unsigned long long* hash;  // FNV-1a of every name, sorted ascending
-    const uint32_t* hash_id;      // name id of the k-th sorted hash
-    uint32_t n_names;
-};
-
 __device__ __forceinline__ bool is_digit(char c) { return c >= '0' && c <= '9'; }
 
 // str::parse::<u32>(): optional '+', at least one digit, digits only, no overflow
@@ -203,7 +195,10 @@ __global__ void ingest_gather_kernel(uint32_t n, const uint32_t* __restrict__ or
 __device__ __forceinline__ bool is_space(char c) { return c == ' ' || (c >= '\t' && c <= '\r'); }  // ASCII White_Space
 
 // One thread per line: '#' lines are skipped; split_whitespace must give at least 5 fields (chr start end barcode ...),
-// start and end parse as u32.  The barcode is carried as (FNV-1a hash, byte span).
+// start and end parse as u32 — and with SUPPORT the fifth field too (Fragment::from_str, gtars-core/src/models/fragments.rs:16-44,
+// which gtars-scoring reads through).  With BARCODE the barcode is carried as (FNV-1a hash, byte span); the count-matrix
+// parse has no use for it and skips the hashing.
+template <bool SUPPORT, bool BARCODE>
 __global__ void ingest_parse_fragments_kernel(uint32_t n_lines, uint32_t n_newlines, uint64_t n_bytes, const char* __restrict__ text,
                                               const uint32_t* __restrict__ nl_pos, NameTable names, uint32_t* __restrict__ keep,
                                               uint32_t* __restrict__ chr, uint32_t* __restrict__ start, uint32_t* __restrict__ end,
@@ -214,7 +209,7 @@ __global__ void ingest_parse_fragments_kernel(uint32_t n_lines, uint32_t n_newli
         uint32_t a = li ? nl_pos[li - 1] + 1 : 0;
         uint32_t b = li < n_newlines ? nl_pos[li] : (uint32_t)n_bytes;
         if (li < n_newlines && b > a && text[b - 1] == '\r') --b;  // only a '\r' in front of a '\n' is part of the line ending
-        uint32_t k = 0, c = GTGPU_UNKNOWN_CHROM, s = 0, e = 0, bo = 0, bl = 0;
+        uint32_t k = 0, c = GTGPU_UNKNOWN_CHROM, s = 0, e = 0, bo = 0, bl = 0, sup = 0;
         unsigned long long h = 1469598103934665603ull;
         if (!(b > a && text[a] == '#')) {
             uint32_t fa[5], fb[5], nf = 0, p = a;
@@ -225,7 +220,8 @@ __global__ void ingest_parse_fragments_kernel(uint32_t n_lines, uint32_t n_newli
                 while (p < b && !is_space(text[p])) ++p;
                 fb[nf++] = p;
             }
-            if (nf < 5 || !parse_u32_field(text, fa[1], fb[1], s) || !parse_u32_field(text, fa[2], fb[2], e)) {
+            if (nf < 5 || !parse_u32_field(text, fa[1], fb[1], s) || !parse_u32_field(text, fa[2], fb[2], e) ||
+                (SUPPORT && !parse_u32_field(text, fa[4], fb[4], sup))) {
                 k = 2;
             } else {
                 k = 1;
@@ -243,10 +239,12 @@ __global__ void ingest_parse_fragments_kernel(uint32_t n_lines, uint32_t n_newli
                     for (uint32_t i = 0; same && i < nb - na; ++i) same = names.blob[na + i] == text[fa[0] + i];
                     if (same) { c = id; break; }
                 }
-                bo = fa[3];
-                bl = fb[3] - fa[3];
-                for (uint32_t i = fa[3]; i < fb[3]; ++i) h = (h ^ (unsigned char)text[i]) * 1099511628211ull;
-                if (h == 0) h = 1;  // 0 marks an empty slot of the barcode table
+                if (BARCODE) {
+                    bo = fa[3];
+                    bl = fb[3] - fa[3];
+                    for (uint32_t i = fa[3]; i < fb[3]; ++i) h = (h ^ (unsigned char)text[i]) * 1099511628211ull;
+                    if (h == 0) h = 1;  // 0 marks an empty slot of the barcode table
+                }
             }
         }
         if (k == 2) atomicMin(first_bad_line, li);
@@ -254,9 +252,11 @@ __global__ void ingest_parse_fragments_kernel(uint32_t n_lines, uint32_t n_newli
         chr[li] = c;
         start[li] = s;
         end[li] = e;
-        bc_hash[li] = h;
-        bc_off[li] = bo;
-        bc_len[li] = bl;
+        if (BARCODE) {
+            bc_hash[li] = h;
+            bc_off[li] = bo;
+            bc_len[li] = bl;
+        }
     }
 }
 
@@ -273,17 +273,19 @@ __global__ void ingest_compact_fragments_kernel(uint32_t n_lines, const uint32_t
             o_chr[p] = chr[i];
             o_start[p] = start[i];
             o_end[p] = end[i];
-            o_h[p] = h[i];
-            o_bo[p] = bo[i];
-            o_bl[p] = bl[i];
+            if (o_h) {  // uniform per launch: the count-matrix parse carries no barcodes
+                o_h[p] = h[i];
+                o_bo[p] = bo[i];
+                o_bl[p] = bl[i];
+            }
         }
 }
 
 // Barcode table (open addressing on the 64-bit hash): every fragment finds or claims its barcode's slot and lowers the
-// slot's first-appearance index to its own position.
+// slot's first-appearance index to its own position, base + k (base = fragments of the file before this window).
 __global__ void ingest_barcode_insert_kernel(uint32_t n, const unsigned long long* __restrict__ h, uint32_t mask,
                                              unsigned long long* __restrict__ keys, uint32_t* __restrict__ first,
-                                             uint32_t* __restrict__ slot_of) {
+                                             uint32_t* __restrict__ slot_of, uint32_t base) {
     const uint32_t stride = gridDim.x * blockDim.x;
     for (uint32_t k = blockIdx.x * blockDim.x + threadIdx.x; k < n; k += stride) {
         const unsigned long long key = h[k];
@@ -293,7 +295,7 @@ __global__ void ingest_barcode_insert_kernel(uint32_t n, const unsigned long lon
             if (prev == 0ull || prev == key) break;
             slot = (slot + 1) & mask;
         }
-        atomicMin(first + slot, k);
+        atomicMin(first + slot, base + k);
         slot_of[k] = slot;
     }
 }
@@ -330,8 +332,224 @@ __global__ void ingest_barcode_ids_kernel(uint32_t n, const uint32_t* __restrict
     }
 }
 
+// ---- the barcode table of the scoring entry points: one table over all windows of a file -----------------------------------
+// A window's fragments are numbered file-wide (base + k), so a slot's first-appearance index is the file-wide index of the
+// barcode's first fragment.  Per fragment the table keeps fidx (that index), per barcode (at its first fragment g) hlen[g]
+// (its byte length) and known[g] (seen on a chromosome of the name table); the bytes go to an arena in the window that
+// first sees the barcode, in first-appearance order, because the text of a plain-text window leaves the device with it.
+__global__ void ingest_barcode_rehash_kernel(uint64_t old_cap, const unsigned long long* __restrict__ okeys,
+                                             const uint32_t* __restrict__ ofirst, const unsigned long long* __restrict__ osoff,
+                                             uint32_t mask, unsigned long long* __restrict__ keys, uint32_t* __restrict__ first,
+                                             unsigned long long* __restrict__ soff) {
+    const uint64_t stride = (uint64_t)gridDim.x * blockDim.x;
+    for (uint64_t s = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x; s < old_cap; s += stride) {
+        const unsigned long long key = okeys[s];
+        if (!key) continue;
+        uint32_t slot = (uint32_t)((key * 0x9E3779B97F4A7C15ull) >> 32) & mask;
+        while (atomicCAS(keys + slot, 0ull, key) != 0ull) slot = (slot + 1) & mask;  // keys are distinct
+        first[slot] = ofirst[s];
+        soff[slot] = osoff[s];
+    }
+}
+
+__global__ void ingest_barcode_window_heads_kernel(uint32_t n, uint32_t base, const uint32_t* __restrict__ slot_of,
+                                                   const uint32_t* __restrict__ first, const uint32_t* __restrict__ chr,
+                                                   const uint32_t* __restrict__ bl, uint32_t n_names, uint32_t* __restrict__ fidx,
+                                                   uint32_t* __restrict__ hlen, uint32_t* __restrict__ known, uint32_t* __restrict__ n_new) {
+    const uint32_t stride = gridDim.x * blockDim.x;
+    for (uint32_t k = blockIdx.x * blockDim.x + threadIdx.x; k < n; k += stride) {
+        const uint32_t f = first[slot_of[k]], g = base + k;
+        const bool head = f == g;
+        fidx[g] = f;
+        hlen[g] = head ? bl[k] : 0u;
+        if (chr[k] < n_names) known[f] = 1u;  // files.rs:106-129: a consensus chromosome creates the barcode's entry
+        const unsigned m = __ballot_sync(__activemask(), head);
+        if (head && (threadIdx.x & 31) == (unsigned)(__ffs(m) - 1)) atomicAdd(n_new, (uint32_t)__popc(m));
+    }
+}
+
+__global__ void ingest_barcode_claim_kernel(uint32_t n, uint32_t base, const char* __restrict__ text, const uint32_t* __restrict__ slot_of,
+                                            const uint32_t* __restrict__ fidx, const uint32_t* __restrict__ bo,
+                                            const uint32_t* __restrict__ bl, const uint32_t* __restrict__ wpos, uint64_t used,
+                                            char* __restrict__ arena, unsigned long long* __restrict__ soff) {
+    const uint32_t stride = gridDim.x * blockDim.x;
+    for (uint32_t k = blockIdx.x * blockDim.x + threadIdx.x; k < n; k += stride) {
+        if (fidx[base + k] != base + k) continue;
+        const uint64_t p = used + wpos[k];
+        for (uint32_t i = 0; i < bl[k]; ++i) arena[p + i] = text[bo[k] + i];
+        soff[slot_of[k]] = p;
+    }
+}
+
+// every later fragment of a barcode has its first appearance's bytes (a 64-bit hash collision would merge two barcodes)
+__global__ void ingest_barcode_check_kernel(uint32_t n, uint32_t base, const char* __restrict__ text, const uint32_t* __restrict__ slot_of,
+                                            const uint32_t* __restrict__ fidx, const uint32_t* __restrict__ bo,
+                                            const uint32_t* __restrict__ bl, const uint32_t* __restrict__ hlen,
+                                            const char* __restrict__ arena, const unsigned long long* __restrict__ soff,
+                                            uint32_t* __restrict__ collision) {
+    const uint32_t stride = gridDim.x * blockDim.x;
+    for (uint32_t k = blockIdx.x * blockDim.x + threadIdx.x; k < n; k += stride) {
+        const uint32_t f = fidx[base + k];
+        if (f == base + k) continue;
+        const uint64_t p = soff[slot_of[k]];
+        bool same = hlen[f] == bl[k];
+        for (uint32_t i = 0; same && i < bl[k]; ++i) same = arena[p + i] == text[bo[k] + i];
+        if (!same) *collision = 1;
+    }
+}
+
+// after the last window: a barcode is kept when it was seen on a known chromosome; alen / klen are the byte lengths of every
+// first appearance / of the kept ones (u64 for the scans)
+__global__ void ingest_barcode_keep_kernel(uint64_t n, const uint32_t* __restrict__ fidx, const uint32_t* __restrict__ known,
+                                           const uint32_t* __restrict__ hlen, uint32_t* __restrict__ keep,
+                                           unsigned long long* __restrict__ alen, unsigned long long* __restrict__ klen) {
+    const uint64_t stride = (uint64_t)gridDim.x * blockDim.x;
+    for (uint64_t g = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x; g < n; g += stride) {
+        const bool kp = fidx[g] == g && known[g];
+        keep[g] = kp;
+        alen[g] = hlen[g];
+        klen[g] = kp ? hlen[g] : 0u;
+    }
+}
+
+// dense ids in first-appearance order among the kept barcodes; a fragment of a dropped barcode lies on an unknown chromosome
+// (it has no hit), so any valid id serves it.  The kept names are gathered from the arena in id order.
+__global__ void ingest_barcode_final_kernel(uint64_t n, const uint32_t* __restrict__ fidx, const uint32_t* __restrict__ keep,
+                                            const uint32_t* __restrict__ rank, const unsigned long long* __restrict__ aoff,
+                                            const unsigned long long* __restrict__ boff, const uint32_t* __restrict__ hlen,
+                                            const char* __restrict__ arena, char* __restrict__ blob,
+                                            unsigned long long* __restrict__ name_off, uint32_t* __restrict__ bc) {
+    const uint64_t stride = (uint64_t)gridDim.x * blockDim.x;
+    for (uint64_t g = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x; g < n; g += stride) {
+        const uint32_t f = fidx[g];
+        bc[g] = keep[f] ? rank[f] : 0u;
+        if (keep[g]) {
+            for (uint32_t i = 0; i < hlen[g]; ++i) blob[boff[g] + i] = arena[aoff[g] + i];
+            name_off[rank[g]] = boff[g];
+        }
+    }
+}
+
 static int igrid(gtgpu_ctx* ctx, uint64_t n) {
     return (int)std::max<uint64_t>(1, std::min<uint64_t>((n + 255) / 256, (uint64_t)ctx->sm_count * 16));
+}
+
+// Fragment name table in scratch SC_SET_ID: FNV-1a hashes of the caller's chromosome names, sorted for the device lookup.
+int32_t upload_name_table(gtgpu_ctx* ctx, uint32_t n_names, const char* names, const uint32_t* name_offsets, NameTable* out) {
+    cudaStream_t st = ctx->stream;
+    std::vector<unsigned long long> hash(n_names), hash_sorted(n_names);
+    std::vector<uint32_t> hash_id(n_names);
+    for (uint32_t i = 0; i < n_names; ++i) {
+        unsigned long long h = 1469598103934665603ull;
+        for (uint32_t k = name_offsets[i]; k < name_offsets[i + 1]; ++k) h = (h ^ (unsigned char)names[k]) * 1099511628211ull;
+        hash[i] = h;
+    }
+    std::iota(hash_id.begin(), hash_id.end(), 0u);
+    std::sort(hash_id.begin(), hash_id.end(), [&](uint32_t a, uint32_t b) { return hash[a] != hash[b] ? hash[a] < hash[b] : a < b; });
+    for (uint32_t i = 0; i < n_names; ++i) hash_sorted[i] = hash[hash_id[i]];
+    const uint32_t blob_bytes = n_names ? name_offsets[n_names] : 0;
+    char* d_names;
+    GT_TRY(ctx->scratch_get(SC_SET_ID, (size_t)n_names * 16 + ((size_t)n_names + 1) * 4 + blob_bytes + 64, (void**)&d_names));
+    unsigned long long* d_hash = reinterpret_cast<unsigned long long*>(d_names);
+    uint32_t* d_noff = reinterpret_cast<uint32_t*>(d_hash + n_names);
+    uint32_t* d_hid = d_noff + n_names + 1;
+    char* d_blob = reinterpret_cast<char*>(d_hid + n_names);
+    if (n_names) {
+        GT_CUDA(cudaMemcpyAsync(d_hash, hash_sorted.data(), (size_t)n_names * 8, cudaMemcpyHostToDevice, st));
+        GT_CUDA(cudaMemcpyAsync(d_hid, hash_id.data(), (size_t)n_names * 4, cudaMemcpyHostToDevice, st));
+        if (blob_bytes) GT_CUDA(cudaMemcpyAsync(d_blob, names, blob_bytes, cudaMemcpyHostToDevice, st));
+    }
+    GT_CUDA(cudaMemcpyAsync(d_noff, name_offsets ? name_offsets : (const uint32_t*)&blob_bytes, ((size_t)n_names + 1) * 4,
+                            cudaMemcpyHostToDevice, st));
+    GT_CUDA(cudaStreamSynchronize(st));  // the host vectors above are pageable and go out of scope
+    *out = NameTable{d_blob, d_noff, d_hash, d_hid, n_names};
+    return GTGPU_OK;
+}
+
+// The fragment front end shared by tokenize_fragment_file and the scoring entry points: newline positions, one thread per
+// line, compaction of the kept lines.  d_text: 0 < n_bytes < 0xFFFFFFF0 bytes of device text, 16-byte aligned.
+int32_t parse_fragments_locked(gtgpu_ctx* ctx, const char* d_text, uint64_t n_bytes, const NameTable& nt, FragMode mode,
+                               FragParse* out) {
+    cudaStream_t st = ctx->stream;
+    uint32_t *d_counts, *d_crank, *d_nl;
+    void* d_tmp;
+    const uint64_t n_chunks = (n_bytes + INGEST_CHUNK - 1) / INGEST_CHUNK;
+    GT_TRY(ctx->scratch_get(SC_COUNTS, n_chunks * 4 + 4, (void**)&d_counts));
+    GT_TRY(ctx->scratch_get(SC_IN3_CHR, n_chunks * 4 + 4, (void**)&d_crank));
+    // ---- lines -------------------------------------------------------------------------------------------------------------
+    GT_TRY(ctx->scratch_get(SC_IN3_START, exclusive_scan_temp_bytes(n_chunks, 4), &d_tmp));
+    ingest_count_newlines_kernel<<<igrid(ctx, n_chunks), 256, 0, st>>>(n_bytes, d_text, d_counts);
+    ctx->launches++;
+    GT_TRY(exclusive_scan<uint32_t>(ctx, d_counts, d_crank, n_chunks, d_tmp));
+    uint32_t last[2];
+    GT_CUDA(cudaMemcpyAsync(&last[0], d_crank + n_chunks - 1, 4, cudaMemcpyDeviceToHost, st));
+    GT_CUDA(cudaMemcpyAsync(&last[1], d_counts + n_chunks - 1, 4, cudaMemcpyDeviceToHost, st));
+    char last_byte = 0;  // read back from the device: with device-resident text there is no host copy
+    GT_CUDA(cudaMemcpyAsync(&last_byte, d_text + n_bytes - 1, 1, cudaMemcpyDeviceToHost, st));
+    GT_CUDA(cudaStreamSynchronize(st));
+    const uint32_t n_newlines = last[0] + last[1];
+    const uint32_t n_lines = n_newlines + (last_byte != '\n' ? 1u : 0u);
+    GT_TRY(ctx->scratch_get(SC_IN3_END, (size_t)n_newlines * 4 + 4, (void**)&d_nl));
+    ingest_newline_positions_kernel<<<igrid(ctx, n_chunks), 256, 0, st>>>(n_bytes, d_text, d_crank, d_nl);
+    ctx->launches++;
+    // ---- parse + compact ---------------------------------------------------------------------------------------------------
+    const bool bc = mode != FRAG_SCORE_MATRIX;
+    const size_t lb = (size_t)n_lines * 4 + 8;
+    uint32_t *d_keep, *d_pos, *p_chr, *p_start, *p_end, *p_bo = nullptr, *p_bl = nullptr, *o_chr, *o_start, *o_end, *o_bo = nullptr,
+             *o_bl = nullptr;
+    unsigned long long *p_h = nullptr, *o_h = nullptr;
+    uint64_t* d_misc;
+    GT_TRY(ctx->scratch_get(SC_IN3_START, exclusive_scan_temp_bytes(n_lines, 4), &d_tmp));
+    GT_TRY(ctx->scratch_get(SC_ING_0, lb, (void**)&d_keep));
+    GT_TRY(ctx->scratch_get(SC_ING_1, lb, (void**)&d_pos));
+    GT_TRY(ctx->scratch_get(SC_IN2_CHR, lb, (void**)&p_chr));
+    GT_TRY(ctx->scratch_get(SC_IN2_START, lb, (void**)&p_start));
+    GT_TRY(ctx->scratch_get(SC_IN2_END, lb, (void**)&p_end));
+    GT_TRY(ctx->scratch_get(SC_CHR, lb, (void**)&o_chr));
+    GT_TRY(ctx->scratch_get(SC_START, lb, (void**)&o_start));
+    GT_TRY(ctx->scratch_get(SC_END, lb, (void**)&o_end));
+    if (bc) {
+        GT_TRY(ctx->scratch_get(SC_ING_2, lb * 2, (void**)&p_h));
+        GT_TRY(ctx->scratch_get(SC_ING_3, lb, (void**)&p_bo));
+        GT_TRY(ctx->scratch_get(SC_ING_4, lb, (void**)&p_bl));
+        GT_TRY(ctx->scratch_get(SC_ING_5, lb * 2, (void**)&o_h));
+        GT_TRY(ctx->scratch_get(SC_ING_6, lb, (void**)&o_bo));
+        GT_TRY(ctx->scratch_get(SC_ING_7, lb, (void**)&o_bl));
+    }
+    GT_TRY(ctx->scratch_get(SC_MISC, 64, (void**)&d_misc));
+    uint32_t* d_flags = reinterpret_cast<uint32_t*>(d_misc);  // [0] first malformed line, [1..3] for the caller's barcode table
+    const uint32_t init[4] = {0xFFFFFFFFu, 0u, 0u, 0u};
+    GT_CUDA(cudaMemcpyAsync(d_flags, init, 16, cudaMemcpyHostToDevice, st));
+    auto kern = mode == FRAG_TOKENIZE ? ingest_parse_fragments_kernel<false, true>
+                : mode == FRAG_SCORE_MATRIX ? ingest_parse_fragments_kernel<true, false> : ingest_parse_fragments_kernel<true, true>;
+    kern<<<igrid(ctx, n_lines), 256, 0, st>>>(n_lines, n_newlines, n_bytes, d_text, d_nl, nt, d_keep, p_chr, p_start, p_end, p_h, p_bo,
+                                              p_bl, d_flags);
+    ctx->launches++;
+    GT_TRY(exclusive_scan<uint32_t>(ctx, d_keep, d_pos, n_lines, d_tmp));
+    ingest_compact_fragments_kernel<<<igrid(ctx, n_lines), 256, 0, st>>>(n_lines, d_keep, d_pos, p_chr, p_start, p_end, p_h, p_bo, p_bl,
+                                                                         o_chr, o_start, o_end, o_h, o_bo, o_bl);
+    ctx->launches++;
+    uint32_t tail[2], flags[1];
+    GT_CUDA(cudaMemcpyAsync(&tail[0], d_pos + n_lines - 1, 4, cudaMemcpyDeviceToHost, st));
+    GT_CUDA(cudaMemcpyAsync(&tail[1], d_keep + n_lines - 1, 4, cudaMemcpyDeviceToHost, st));
+    GT_CUDA(cudaMemcpyAsync(flags, d_flags, 4, cudaMemcpyDeviceToHost, st));
+    GT_CUDA(cudaStreamSynchronize(st));
+    *out = FragParse{};
+    out->n_lines = n_lines;
+    out->bad_line = flags[0];
+    out->n = flags[0] == 0xFFFFFFFFu ? tail[0] + tail[1] : 0;
+    out->chr = o_chr;
+    out->start = o_start;
+    out->end = o_end;
+    out->h = o_h;
+    out->bo = o_bo;
+    out->bl = o_bl;
+    out->free0 = d_keep;  // the line-sized arrays are free again
+    out->free1 = d_pos;
+    out->free2 = p_chr;
+    out->tmp = d_tmp;
+    out->flags = d_flags;
+    return GTGPU_OK;
 }
 
 // Parses and sorts on the device.  On success *d_chr / *d_start / *d_end point at n_out regions in device scratch
@@ -475,6 +693,157 @@ static int32_t parse_bed_locked(gtgpu_ctx* ctx, const char* text, uint64_t n_byt
     return GTGPU_OK;
 }
 
+int32_t DevMem::reserve(size_t bytes, size_t keep, cudaStream_t st) {
+    if (cap >= bytes) return GTGPU_OK;
+    void* p = nullptr;
+    size_t want = std::max(bytes, cap + cap / 2);
+    if (cudaMalloc(&p, want) != cudaSuccess) {
+        cudaGetLastError();
+        want = bytes;
+        cudaError_t e = cudaMalloc(&p, want);
+        if (e != cudaSuccess) return fail(GTGPU_ERR_NOMEM, "cudaMalloc(" + std::to_string(bytes) + " B): " + cudaGetErrorString(e));
+    }
+    if (keep) GT_CUDA(cudaMemcpyAsync(p, ptr, keep, cudaMemcpyDeviceToDevice, st));
+    GT_CUDA(cudaStreamSynchronize(st));
+    if (ptr) cudaFree(ptr);
+    ptr = p;
+    cap = want;
+    return GTGPU_OK;
+}
+
+DevMem::~DevMem() {
+    if (ptr) cudaFree(ptr);
+}
+
+int32_t FragBarcodeTable::add_window(gtgpu_ctx* ctx, const char* d_text, const FragParse& fp, uint32_t n_names) {
+    const uint32_t nw = fp.n;
+    if (nw == 0) return GTGPU_OK;
+    cudaStream_t st = ctx->stream;
+    const uint32_t base = (uint32_t)n;
+    const size_t need = (size_t)(n + nw) * 4, have = (size_t)n * 4;
+    for (DevMem* m : {&chr, &start, &end, &fidx, &known, &hlen}) GT_TRY(m->reserve(need, have, st));
+    GT_CUDA(cudaMemcpyAsync(chr.u32() + base, fp.chr, (size_t)nw * 4, cudaMemcpyDeviceToDevice, st));
+    GT_CUDA(cudaMemcpyAsync(start.u32() + base, fp.start, (size_t)nw * 4, cudaMemcpyDeviceToDevice, st));
+    GT_CUDA(cudaMemcpyAsync(end.u32() + base, fp.end, (size_t)nw * 4, cudaMemcpyDeviceToDevice, st));
+    GT_CUDA(cudaMemsetAsync(known.u32() + base, 0, (size_t)nw * 4, st));
+    // the table holds at most distinct + nw barcodes after this window: keep it at most half full
+    uint64_t new_cap = std::max<uint64_t>(cap, 1024);
+    while (new_cap < 2 * (distinct + nw)) new_cap <<= 1;
+    if (new_cap != cap) {
+        DevMem k2, f2, s2;
+        GT_TRY(k2.reserve(new_cap * 8, 0, st));
+        GT_TRY(f2.reserve(new_cap * 4, 0, st));
+        GT_TRY(s2.reserve(new_cap * 8, 0, st));
+        GT_CUDA(cudaMemsetAsync(k2.ptr, 0, new_cap * 8, st));
+        GT_CUDA(cudaMemsetAsync(f2.ptr, 0xFF, new_cap * 4, st));
+        if (cap) {
+            ingest_barcode_rehash_kernel<<<igrid(ctx, cap), 256, 0, st>>>(cap, (const unsigned long long*)keys.ptr, first.u32(),
+                                                                         (const unsigned long long*)soff.ptr, (uint32_t)(new_cap - 1),
+                                                                         (unsigned long long*)k2.ptr, f2.u32(), (unsigned long long*)s2.ptr);
+            ctx->launches++;
+        }
+        GT_CUDA(cudaStreamSynchronize(st));
+        keys.swap(k2);
+        first.swap(f2);
+        soff.swap(s2);
+        cap = new_cap;
+    }
+    uint32_t* slot_of = fp.free0;
+    uint32_t* wpos = fp.free1;
+    ingest_barcode_insert_kernel<<<igrid(ctx, nw), 256, 0, st>>>(nw, fp.h, (uint32_t)(cap - 1), (unsigned long long*)keys.ptr, first.u32(),
+                                                                 slot_of, base);
+    ingest_barcode_window_heads_kernel<<<igrid(ctx, nw), 256, 0, st>>>(nw, base, slot_of, first.u32(), fp.chr, fp.bl, n_names, fidx.u32(),
+                                                                       hlen.u32(), known.u32(), fp.flags + 2);
+    ctx->launches += 2;
+    GT_TRY(exclusive_scan<uint32_t>(ctx, hlen.u32() + base, wpos, nw, fp.tmp));
+    uint32_t tail[3];
+    GT_CUDA(cudaMemcpyAsync(&tail[0], wpos + nw - 1, 4, cudaMemcpyDeviceToHost, st));
+    GT_CUDA(cudaMemcpyAsync(&tail[1], hlen.u32() + base + nw - 1, 4, cudaMemcpyDeviceToHost, st));
+    GT_CUDA(cudaMemcpyAsync(&tail[2], fp.flags + 2, 4, cudaMemcpyDeviceToHost, st));
+    GT_CUDA(cudaStreamSynchronize(st));
+    const uint64_t bytes = (uint64_t)tail[0] + tail[1];
+    GT_TRY(arena.reserve(used + bytes + 1, used, st));
+    ingest_barcode_claim_kernel<<<igrid(ctx, nw), 256, 0, st>>>(nw, base, d_text, slot_of, fidx.u32(), fp.bo, fp.bl, wpos, used,
+                                                                (char*)arena.ptr, (unsigned long long*)soff.ptr);
+    ingest_barcode_check_kernel<<<igrid(ctx, nw), 256, 0, st>>>(nw, base, d_text, slot_of, fidx.u32(), fp.bo, fp.bl, hlen.u32(),
+                                                                (const char*)arena.ptr, (const unsigned long long*)soff.ptr, fp.flags + 1);
+    ctx->launches += 2;
+    uint32_t collision = 0;
+    GT_CUDA(cudaMemcpyAsync(&collision, fp.flags + 1, 4, cudaMemcpyDeviceToHost, st));
+    GT_CUDA(cudaStreamSynchronize(st));  // the window's text may be overwritten after this
+    if (collision) return fail(GTGPU_ERR_UNSUPPORTED, "two barcodes share a 64-bit hash; use gtgpu_score_barcodes");
+    used += bytes;
+    distinct += tail[2];
+    n += nw;
+    return GTGPU_OK;
+}
+
+int32_t FragBarcodeTable::finish(gtgpu_ctx* ctx, uint32_t* n_kept, gtgpu_buf** out_names, gtgpu_buf** out_name_offsets) {
+    cudaStream_t st = ctx->stream;
+    uint64_t kept = 0, blob_bytes = 0;
+    char* d_blob = nullptr;
+    unsigned long long* d_noff = nullptr;
+    if (n) {
+        uint32_t *d_keep, *d_rank;
+        unsigned long long *d_alen, *d_klen, *d_aoff, *d_boff;
+        void* d_tmp;
+        GT_TRY(ctx->scratch_get(SC_ING_0, n * 4, (void**)&d_keep));
+        GT_TRY(ctx->scratch_get(SC_ING_1, n * 4, (void**)&d_rank));
+        GT_TRY(ctx->scratch_get(SC_ING_2, n * 8, (void**)&d_alen));
+        GT_TRY(ctx->scratch_get(SC_ING_5, n * 8, (void**)&d_klen));
+        GT_TRY(ctx->scratch_get(SC_ING_3, n * 8, (void**)&d_aoff));
+        GT_TRY(ctx->scratch_get(SC_ING_4, n * 8, (void**)&d_boff));
+        GT_TRY(ctx->scratch_get(SC_IN3_START, exclusive_scan_temp_bytes(n, 8), &d_tmp));
+        GT_TRY(bc.reserve(n * 4, 0, st));
+        ingest_barcode_keep_kernel<<<igrid(ctx, n), 256, 0, st>>>(n, fidx.u32(), known.u32(), hlen.u32(), d_keep, d_alen, d_klen);
+        ctx->launches++;
+        GT_TRY(exclusive_scan<uint32_t>(ctx, d_keep, d_rank, n, d_tmp));
+        GT_TRY(exclusive_scan<unsigned long long>(ctx, d_alen, d_aoff, n, d_tmp));
+        GT_TRY(exclusive_scan<unsigned long long>(ctx, d_klen, d_boff, n, d_tmp));
+        uint32_t t32[2];
+        unsigned long long t64[2];
+        GT_CUDA(cudaMemcpyAsync(&t32[0], d_rank + n - 1, 4, cudaMemcpyDeviceToHost, st));
+        GT_CUDA(cudaMemcpyAsync(&t32[1], d_keep + n - 1, 4, cudaMemcpyDeviceToHost, st));
+        GT_CUDA(cudaMemcpyAsync(&t64[0], d_boff + n - 1, 8, cudaMemcpyDeviceToHost, st));
+        GT_CUDA(cudaMemcpyAsync(&t64[1], d_klen + n - 1, 8, cudaMemcpyDeviceToHost, st));
+        GT_CUDA(cudaStreamSynchronize(st));
+        kept = (uint64_t)t32[0] + t32[1];
+        blob_bytes = t64[0] + t64[1];
+        GT_TRY(ctx->scratch_get(SC_ING_6, blob_bytes + 1, (void**)&d_blob));
+        GT_TRY(ctx->scratch_get(SC_ING_7, (kept + 1) * 8, (void**)&d_noff));
+        ingest_barcode_final_kernel<<<igrid(ctx, n), 256, 0, st>>>(n, fidx.u32(), d_keep, d_rank, d_aoff, d_boff, hlen.u32(),
+                                                                   (const char*)arena.ptr, d_blob, d_noff, bc.u32());
+        ctx->launches++;
+        GT_CUDA(cudaGetLastError());
+    }
+    gtgpu_buf* bufs[2] = {new gtgpu_buf(), new gtgpu_buf()};
+    const uint64_t lens[2] = {blob_bytes, kept + 1};
+    int32_t s = GTGPU_OK;
+    for (int k = 0; k < 2; ++k) {
+        bufs[k]->ctx = ctx;
+        bufs[k]->len = lens[k];
+        bufs[k]->elem_size = k == 0 ? 1 : 8;
+        if (s == GTGPU_OK) s = ctx->pinned_get(lens[k] * bufs[k]->elem_size, &bufs[k]->block);
+    }
+    if (s == GTGPU_OK && blob_bytes && cudaMemcpyAsync(bufs[0]->block.ptr, d_blob, blob_bytes, cudaMemcpyDeviceToHost, st) != cudaSuccess)
+        s = fail(GTGPU_ERR_CUDA, "score_barcodes_text: D2H of the barcode names failed");
+    if (s == GTGPU_OK && kept && cudaMemcpyAsync(bufs[1]->block.ptr, d_noff, kept * 8, cudaMemcpyDeviceToHost, st) != cudaSuccess)
+        s = fail(GTGPU_ERR_CUDA, "score_barcodes_text: D2H of the barcode name offsets failed");
+    if (s == GTGPU_OK && cudaStreamSynchronize(st) != cudaSuccess) s = fail(GTGPU_ERR_CUDA, "score_barcodes_text: D2H failed");
+    if (s != GTGPU_OK) {
+        for (auto* b : bufs) {
+            if (b->block.ptr) ctx->pinned_put(b->block);
+            delete b;
+        }
+        return s;
+    }
+    reinterpret_cast<uint64_t*>(bufs[1]->block.ptr)[kept] = blob_bytes;
+    *n_kept = (uint32_t)kept;
+    *out_names = bufs[0];
+    *out_name_offsets = bufs[1];
+    return GTGPU_OK;
+}
+
 static int32_t to_host_buf(gtgpu_ctx* ctx, const uint32_t* d_src, uint64_t n, gtgpu_buf** out) {
     gtgpu_buf* buf = new gtgpu_buf();
     buf->ctx = ctx;
@@ -586,118 +955,44 @@ int32_t gtgpu::tokenize_fragments_text_locked(gtgpu_index* ix, const char* text,
     uint32_t n = 0, n_barcodes = 0;
     uint32_t *o_chr = nullptr, *o_start = nullptr, *o_end = nullptr, *d_bcid = nullptr, *d_spans = nullptr;
     if (n_bytes) {
-        // ---- name table (as in parse_bed_locked) -------------------------------------------------------------------------
-        std::vector<unsigned long long> hash(n_names), hash_sorted(n_names);
-        std::vector<uint32_t> hash_id(n_names);
-        for (uint32_t i = 0; i < n_names; ++i) {
-            unsigned long long h = 1469598103934665603ull;
-            for (uint32_t k = name_offsets[i]; k < name_offsets[i + 1]; ++k) h = (h ^ (unsigned char)names[k]) * 1099511628211ull;
-            hash[i] = h;
-        }
-        std::iota(hash_id.begin(), hash_id.end(), 0u);
-        std::sort(hash_id.begin(), hash_id.end(), [&](uint32_t a, uint32_t b) { return hash[a] != hash[b] ? hash[a] < hash[b] : a < b; });
-        for (uint32_t i = 0; i < n_names; ++i) hash_sorted[i] = hash[hash_id[i]];
-        const uint32_t blob_bytes = n_names ? name_offsets[n_names] : 0;
-        char *d_text, *d_names;
-        uint32_t *d_counts, *d_crank, *d_nl;
-        void* d_tmp;
-        const uint64_t n_chunks = (n_bytes + INGEST_CHUNK - 1) / INGEST_CHUNK;
+        NameTable nt;
+        GT_TRY(upload_name_table(ctx, n_names, names, name_offsets, &nt));
+        char* d_text;
         if (ctx->ingest_d_text) d_text = (char*)ctx->ingest_d_text;
         else GT_TRY(ctx->scratch_get(SC_OUT_IDS2, n_bytes + 64, (void**)&d_text));
-        GT_TRY(ctx->scratch_get(SC_COUNTS, n_chunks * 4 + 4, (void**)&d_counts));
-        GT_TRY(ctx->scratch_get(SC_IN3_CHR, n_chunks * 4 + 4, (void**)&d_crank));
-        GT_TRY(ctx->scratch_get(SC_SET_ID, (size_t)n_names * 16 + ((size_t)n_names + 1) * 4 + blob_bytes + 64, (void**)&d_names));
         if (!ctx->ingest_d_text) GT_CUDA(cudaMemcpyAsync(d_text, text, n_bytes, cudaMemcpyHostToDevice, st));
-        unsigned long long* d_hash = reinterpret_cast<unsigned long long*>(d_names);
-        uint32_t* d_noff = reinterpret_cast<uint32_t*>(d_hash + n_names);
-        uint32_t* d_hid = d_noff + n_names + 1;
-        char* d_blob = reinterpret_cast<char*>(d_hid + n_names);
-        if (n_names) {
-            GT_CUDA(cudaMemcpyAsync(d_hash, hash_sorted.data(), (size_t)n_names * 8, cudaMemcpyHostToDevice, st));
-            GT_CUDA(cudaMemcpyAsync(d_hid, hash_id.data(), (size_t)n_names * 4, cudaMemcpyHostToDevice, st));
-            if (blob_bytes) GT_CUDA(cudaMemcpyAsync(d_blob, names, blob_bytes, cudaMemcpyHostToDevice, st));
-        }
-        GT_CUDA(cudaMemcpyAsync(d_noff, name_offsets ? name_offsets : (const uint32_t*)&blob_bytes, ((size_t)n_names + 1) * 4,
-                                cudaMemcpyHostToDevice, st));
-        // ---- lines -------------------------------------------------------------------------------------------------------------
-        GT_TRY(ctx->scratch_get(SC_IN3_START, exclusive_scan_temp_bytes(n_chunks, 4), &d_tmp));
-        ingest_count_newlines_kernel<<<igrid(ctx, n_chunks), 256, 0, st>>>(n_bytes, d_text, d_counts);
-        ctx->launches++;
-        GT_TRY(exclusive_scan<uint32_t>(ctx, d_counts, d_crank, n_chunks, d_tmp));
-        uint32_t last[2];
-        GT_CUDA(cudaMemcpyAsync(&last[0], d_crank + n_chunks - 1, 4, cudaMemcpyDeviceToHost, st));
-        GT_CUDA(cudaMemcpyAsync(&last[1], d_counts + n_chunks - 1, 4, cudaMemcpyDeviceToHost, st));
-        char last_byte = 0;  // read back from the device: with device-resident text there is no host copy
-        GT_CUDA(cudaMemcpyAsync(&last_byte, d_text + n_bytes - 1, 1, cudaMemcpyDeviceToHost, st));
-        GT_CUDA(cudaStreamSynchronize(st));
-        const uint32_t n_newlines = last[0] + last[1];
-        const uint32_t n_lines = n_newlines + (last_byte != '\n' ? 1u : 0u);
-        GT_TRY(ctx->scratch_get(SC_IN3_END, (size_t)n_newlines * 4 + 4, (void**)&d_nl));
-        ingest_newline_positions_kernel<<<igrid(ctx, n_chunks), 256, 0, st>>>(n_bytes, d_text, d_crank, d_nl);
-        ctx->launches++;
-        // ---- parse + compact ---------------------------------------------------------------------------------------------------
-        const size_t lb = (size_t)n_lines * 4 + 8;
-        uint32_t *d_keep, *d_pos, *p_chr, *p_start, *p_end, *p_bo, *p_bl, *o_bo, *o_bl;
-        unsigned long long *p_h, *o_h;
-        uint64_t* d_misc;
-        GT_TRY(ctx->scratch_get(SC_IN3_START, exclusive_scan_temp_bytes(n_lines, 4), &d_tmp));
-        GT_TRY(ctx->scratch_get(SC_ING_0, lb, (void**)&d_keep));
-        GT_TRY(ctx->scratch_get(SC_ING_1, lb, (void**)&d_pos));
-        GT_TRY(ctx->scratch_get(SC_IN2_CHR, lb, (void**)&p_chr));
-        GT_TRY(ctx->scratch_get(SC_IN2_START, lb, (void**)&p_start));
-        GT_TRY(ctx->scratch_get(SC_IN2_END, lb, (void**)&p_end));
-        GT_TRY(ctx->scratch_get(SC_ING_2, lb * 2, (void**)&p_h));
-        GT_TRY(ctx->scratch_get(SC_ING_3, lb, (void**)&p_bo));
-        GT_TRY(ctx->scratch_get(SC_ING_4, lb, (void**)&p_bl));
-        GT_TRY(ctx->scratch_get(SC_CHR, lb, (void**)&o_chr));
-        GT_TRY(ctx->scratch_get(SC_START, lb, (void**)&o_start));
-        GT_TRY(ctx->scratch_get(SC_END, lb, (void**)&o_end));
-        GT_TRY(ctx->scratch_get(SC_BARCODE, lb, (void**)&d_bcid));
-        GT_TRY(ctx->scratch_get(SC_ING_5, lb * 2, (void**)&o_h));
-        GT_TRY(ctx->scratch_get(SC_ING_6, lb, (void**)&o_bo));
-        GT_TRY(ctx->scratch_get(SC_ING_7, lb, (void**)&o_bl));
-        GT_TRY(ctx->scratch_get(SC_MISC, 64, (void**)&d_misc));
-        uint32_t* d_flags = reinterpret_cast<uint32_t*>(d_misc);  // [0] first malformed line, [1] hash collision
-        const uint32_t init[2] = {0xFFFFFFFFu, 0u};
-        GT_CUDA(cudaMemcpyAsync(d_flags, init, 8, cudaMemcpyHostToDevice, st));
-        NameTable nt{d_blob, d_noff, d_hash, d_hid, n_names};
-        ingest_parse_fragments_kernel<<<igrid(ctx, n_lines), 256, 0, st>>>(n_lines, n_newlines, n_bytes, d_text, d_nl, nt, d_keep, p_chr,
-                                                                           p_start, p_end, p_h, p_bo, p_bl, d_flags);
-        ctx->launches++;
-        GT_TRY(exclusive_scan<uint32_t>(ctx, d_keep, d_pos, n_lines, d_tmp));
-        ingest_compact_fragments_kernel<<<igrid(ctx, n_lines), 256, 0, st>>>(n_lines, d_keep, d_pos, p_chr, p_start, p_end, p_h, p_bo, p_bl,
-                                                                             o_chr, o_start, o_end, o_h, o_bo, o_bl);
-        ctx->launches++;
-        uint32_t tail[2], flags[2];
-        GT_CUDA(cudaMemcpyAsync(&tail[0], d_pos + n_lines - 1, 4, cudaMemcpyDeviceToHost, st));
-        GT_CUDA(cudaMemcpyAsync(&tail[1], d_keep + n_lines - 1, 4, cudaMemcpyDeviceToHost, st));
-        GT_CUDA(cudaMemcpyAsync(flags, d_flags, 4, cudaMemcpyDeviceToHost, st));
-        GT_CUDA(cudaStreamSynchronize(st));
-        if (flags[0] != 0xFFFFFFFFu)
-            return fail(GTGPU_ERR_INVALID, "tokenize_fragments_text: Invalid fragment file detected at line: " + std::to_string(flags[0]));
-        n = tail[0] + tail[1];
+        FragParse fp;
+        GT_TRY(parse_fragments_locked(ctx, d_text, n_bytes, nt, FRAG_TOKENIZE, &fp));
+        if (fp.bad_line != 0xFFFFFFFFu)
+            return fail(GTGPU_ERR_INVALID, "tokenize_fragments_text: Invalid fragment file detected at line: " + std::to_string(fp.bad_line));
+        n = fp.n;
+        o_chr = fp.chr;
+        o_start = fp.start;
+        o_end = fp.end;
         if (n) {
             // ---- barcodes -> dense ids in first-appearance order -----------------------------------------------------------------
             uint64_t cap = 1024;
             while (cap < 2ull * n) cap <<= 1;
             unsigned long long* d_keys;
-            uint32_t *d_first, *d_slot_of = d_keep, *d_head = d_pos, *d_rank = p_chr;  // line-sized arrays are free again
+            uint32_t *d_first, *d_slot_of = fp.free0, *d_head = fp.free1, *d_rank = fp.free2;
+            uint32_t tail[2], flags[2];
+            GT_TRY(ctx->scratch_get(SC_BARCODE, (size_t)n * 4 + 8, (void**)&d_bcid));
             GT_TRY(ctx->scratch_get(SC_MATRIX, cap * 12, (void**)&d_keys));
             d_first = reinterpret_cast<uint32_t*>(d_keys + cap);
             GT_CUDA(cudaMemsetAsync(d_keys, 0, cap * 8, st));
             GT_CUDA(cudaMemsetAsync(d_first, 0xFF, cap * 4, st));
-            ingest_barcode_insert_kernel<<<igrid(ctx, n), 256, 0, st>>>(n, o_h, (uint32_t)(cap - 1), d_keys, d_first, d_slot_of);
-            ingest_barcode_heads_kernel<<<igrid(ctx, n), 256, 0, st>>>(n, d_text, d_slot_of, d_first, o_bo, o_bl, d_head, d_flags + 1);
+            ingest_barcode_insert_kernel<<<igrid(ctx, n), 256, 0, st>>>(n, fp.h, (uint32_t)(cap - 1), d_keys, d_first, d_slot_of, 0u);
+            ingest_barcode_heads_kernel<<<igrid(ctx, n), 256, 0, st>>>(n, d_text, d_slot_of, d_first, fp.bo, fp.bl, d_head, fp.flags + 1);
             ctx->launches += 2;
-            GT_TRY(exclusive_scan<uint32_t>(ctx, d_head, d_rank, n, d_tmp));
+            GT_TRY(exclusive_scan<uint32_t>(ctx, d_head, d_rank, n, fp.tmp));
             GT_CUDA(cudaMemcpyAsync(&tail[0], d_rank + n - 1, 4, cudaMemcpyDeviceToHost, st));
             GT_CUDA(cudaMemcpyAsync(&tail[1], d_head + n - 1, 4, cudaMemcpyDeviceToHost, st));
-            GT_CUDA(cudaMemcpyAsync(flags, d_flags, 8, cudaMemcpyDeviceToHost, st));
+            GT_CUDA(cudaMemcpyAsync(flags, fp.flags, 8, cudaMemcpyDeviceToHost, st));
             GT_CUDA(cudaStreamSynchronize(st));
             if (flags[1]) return fail(GTGPU_ERR_UNSUPPORTED, "tokenize_fragments_text: two barcodes share a 64-bit hash; use the array entry point");
             n_barcodes = tail[0] + tail[1];
             GT_TRY(ctx->scratch_get(SC_FILE_OFFS, (size_t)n_barcodes * 8 + 8, (void**)&d_spans));
-            ingest_barcode_ids_kernel<<<igrid(ctx, n), 256, 0, st>>>(n, d_slot_of, d_first, d_rank, o_bo, o_bl, d_bcid, d_spans);
+            ingest_barcode_ids_kernel<<<igrid(ctx, n), 256, 0, st>>>(n, d_slot_of, d_first, d_rank, fp.bo, fp.bl, d_bcid, d_spans);
             ctx->launches++;
             GT_CUDA(cudaGetLastError());
         }

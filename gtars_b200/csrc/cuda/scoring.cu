@@ -11,6 +11,9 @@
 //   barcodes: fused find with per-fragment offsets -> barcode of every hit -> two stable radix sorts (peak, then
 //             barcode) -> run-length encode -> CSR (barcode offsets, peaks, counts)
 #include <algorithm>
+#include <cstdlib>
+#include <cstring>
+#include <thread>
 
 #include "common.cuh"
 
@@ -138,13 +141,13 @@ int32_t fused_find_all(gtgpu_index* ix, uint64_t nq, uint64_t n_files, const uin
     return GTGPU_OK;
 }
 
-// Device-resident core of gtgpu_score_matrix: d_out_counts (n_files x n_cols u32) is zeroed here.
+// Device-resident core of gtgpu_score_matrix: d_out_counts (n_files x n_cols u32) is zeroed here unless `accumulate`.
 static int32_t score_matrix_dev_locked(gtgpu_index* ix, uint64_t n_files, const uint64_t* d_file_offsets, uint64_t n,
                                        const uint32_t* d_chr, const uint32_t* d_start, const uint32_t* d_end, int32_t mode,
-                                       uint64_t n_cols, uint32_t* d_out_counts) {
+                                       uint64_t n_cols, uint32_t* d_out_counts, bool accumulate = false) {
     gtgpu_ctx* ctx = ix->ctx;
     cudaStream_t st = ctx->stream;
-    GT_CUDA(cudaMemsetAsync(d_out_counts, 0, n_files * n_cols * 4, st));
+    if (!accumulate) GT_CUDA(cudaMemsetAsync(d_out_counts, 0, n_files * n_cols * 4, st));
     if (n == 0 || n_files == 0 || n_cols == 0) return GTGPU_OK;
     const uint32_t *qc = d_chr, *qs = d_start, *qe = d_end;
     const uint64_t* qfo = d_file_offsets;
@@ -259,33 +262,18 @@ extern "C" int32_t gtgpu_score_matrix(gtgpu_index* ix, uint64_t n_files, const u
     return GTGPU_OK;
 } GT_CATCH
 
-extern "C" int32_t gtgpu_score_barcodes(gtgpu_index* ix, uint64_t n, const uint32_t* chr, const uint32_t* start,
-                                        const uint32_t* end, const uint32_t* barcode_id, uint32_t n_barcodes,
-                                        uint64_t* out_barcode_offsets, gtgpu_buf** out_peaks, gtgpu_buf** out_counts) try {
-    if (!ix || !out_barcode_offsets || !out_peaks || !out_counts || (n && (!chr || !start || !end || !barcode_id)))
-        return fail(GTGPU_ERR_INVALID, "score_barcodes: null argument");
-    if (n >= 0xFFFFFFFFull) return fail(GTGPU_ERR_UNSUPPORTED, "score_barcodes: more than 2^32-2 fragments per call");
-    for (uint64_t i = 0; i < n; ++i)
-        if (barcode_id[i] >= n_barcodes) return fail(GTGPU_ERR_INVALID, "score_barcodes: barcode id out of range");
+// Device-resident core of gtgpu_score_barcodes (the caller holds ctx->mu): fragments and dense barcode ids on the device,
+// out_barcode_offsets (n_barcodes + 1) on the host.
+static int32_t score_barcodes_dev_locked(gtgpu_index* ix, uint64_t n, const uint32_t* d_chr, const uint32_t* d_start,
+                                         const uint32_t* d_end, const uint32_t* d_bc, uint32_t n_barcodes,
+                                         uint64_t* out_barcode_offsets, gtgpu_buf** out_peaks, gtgpu_buf** out_counts) {
     gtgpu_ctx* ctx = ix->ctx;
-    std::lock_guard<std::mutex> lk(ctx->mu);
-    GT_CUDA(cudaSetDevice(ctx->device));
     cudaStream_t st = ctx->stream;
-
     uint64_t nnz = 0, total = 0;
     uint32_t *d_peak_out = nullptr, *d_count_out = nullptr;
     if (n) {
-        uint32_t *d_chr, *d_start, *d_end, *d_bc;
         uint64_t* d_off;
-        GT_TRY(ctx->scratch_get(SC_CHR, n * 4, (void**)&d_chr));
-        GT_TRY(ctx->scratch_get(SC_START, n * 4, (void**)&d_start));
-        GT_TRY(ctx->scratch_get(SC_END, n * 4, (void**)&d_end));
-        GT_TRY(ctx->scratch_get(SC_BARCODE, n * 4, (void**)&d_bc));
         GT_TRY(ctx->scratch_get(SC_OUT_OFFS, (n + 1) * 8, (void**)&d_off));
-        GT_CUDA(cudaMemcpyAsync(d_chr, chr, n * 4, cudaMemcpyHostToDevice, st));
-        GT_CUDA(cudaMemcpyAsync(d_start, start, n * 4, cudaMemcpyHostToDevice, st));
-        GT_CUDA(cudaMemcpyAsync(d_end, end, n * 4, cudaMemcpyHostToDevice, st));
-        GT_CUDA(cudaMemcpyAsync(d_bc, barcode_id, n * 4, cudaMemcpyHostToDevice, st));
         uint32_t* d_ids = nullptr;
         GT_TRY(fused_find_all(ix, n, 0, nullptr, d_chr, d_start, d_end, d_off, nullptr, &d_ids, &total));
         if (total >= 0xFFFFFFFFull) return fail(GTGPU_ERR_UNSUPPORTED, "score_barcodes: more than 2^32-2 hits per call");
@@ -361,4 +349,314 @@ extern "C" int32_t gtgpu_score_barcodes(gtgpu_index* ix, uint64_t n, const uint3
     *out_peaks = bufs[0];
     *out_counts = bufs[1];
     return GTGPU_OK;
+}
+
+extern "C" int32_t gtgpu_score_barcodes(gtgpu_index* ix, uint64_t n, const uint32_t* chr, const uint32_t* start,
+                                        const uint32_t* end, const uint32_t* barcode_id, uint32_t n_barcodes,
+                                        uint64_t* out_barcode_offsets, gtgpu_buf** out_peaks, gtgpu_buf** out_counts) try {
+    if (!ix || !out_barcode_offsets || !out_peaks || !out_counts || (n && (!chr || !start || !end || !barcode_id)))
+        return fail(GTGPU_ERR_INVALID, "score_barcodes: null argument");
+    if (n >= 0xFFFFFFFFull) return fail(GTGPU_ERR_UNSUPPORTED, "score_barcodes: more than 2^32-2 fragments per call");
+    for (uint64_t i = 0; i < n; ++i)
+        if (barcode_id[i] >= n_barcodes) return fail(GTGPU_ERR_INVALID, "score_barcodes: barcode id out of range");
+    gtgpu_ctx* ctx = ix->ctx;
+    std::lock_guard<std::mutex> lk(ctx->mu);
+    GT_CUDA(cudaSetDevice(ctx->device));
+    cudaStream_t st = ctx->stream;
+    uint32_t *d_chr = nullptr, *d_start = nullptr, *d_end = nullptr, *d_bc = nullptr;
+    if (n) {
+        GT_TRY(ctx->scratch_get(SC_CHR, n * 4, (void**)&d_chr));
+        GT_TRY(ctx->scratch_get(SC_START, n * 4, (void**)&d_start));
+        GT_TRY(ctx->scratch_get(SC_END, n * 4, (void**)&d_end));
+        GT_TRY(ctx->scratch_get(SC_BARCODE, n * 4, (void**)&d_bc));
+        GT_CUDA(cudaMemcpyAsync(d_chr, chr, n * 4, cudaMemcpyHostToDevice, st));
+        GT_CUDA(cudaMemcpyAsync(d_start, start, n * 4, cudaMemcpyHostToDevice, st));
+        GT_CUDA(cudaMemcpyAsync(d_end, end, n * 4, cudaMemcpyHostToDevice, st));
+        GT_CUDA(cudaMemcpyAsync(d_bc, barcode_id, n * 4, cudaMemcpyHostToDevice, st));
+    }
+    return score_barcodes_dev_locked(ix, n, d_chr, d_start, d_end, d_bc, n_barcodes, out_barcode_offsets, out_peaks, out_counts);
+} GT_CATCH
+
+// ---- region / barcode scoring from a fragment file's bytes -----------------------------------------------------------------
+// The text is parsed in windows (the parse kernels address a window with u32 positions): a window ends right after the first
+// '\n' at or past its nominal size, so it holds whole lines, and a window's local line index plus the lines of the windows
+// before it is the file-wide index the host parser reports.  Plain text is copied window by window (the copy of window k+1,
+// through pinned staging on the copy stream, overlaps the kernels of window k); gzip members are inflated whole into device
+// memory first and the windows run over that text.
+namespace gtgpu {
+
+// GTGPU_INGEST_WINDOW=<bytes>, read per call: nominal window size (results never depend on it)
+static uint64_t ingest_window_bytes() {
+    uint64_t w = 2ull << 30;
+    if (const char* env = getenv("GTGPU_INGEST_WINDOW")) {
+        const uint64_t v = strtoull(env, nullptr, 10);
+        if (v) w = v;
+    }
+    return std::min<uint64_t>(w, 3ull << 30);
+}
+
+using WindowFn = std::function<int32_t(const char* d_window, uint64_t n_bytes, uint64_t first_line, uint32_t* n_lines)>;
+
+struct StagingScope {  // pinned staging blocks and their events, returned to the ctx when the call ends
+    gtgpu_ctx* ctx;
+    PinnedBlock pin[2];
+    cudaEvent_t ev[2] = {nullptr, nullptr};
+    bool used[2] = {false, false};
+    explicit StagingScope(gtgpu_ctx* c) : ctx(c) {}
+    ~StagingScope() {
+        cudaStreamSynchronize(ctx->copy_in);
+        for (int b = 0; b < 2; ++b) {
+            if (ev[b]) cudaEventDestroy(ev[b]);
+            ctx->pinned_put(pin[b]);
+        }
+    }
+};
+
+// Exactly one of host_text / dev_text is given.  The caller holds ctx->mu.
+static int32_t for_each_window(gtgpu_ctx* ctx, const char* host_text, const char* dev_text, uint64_t n_bytes, const std::string& who,
+                               const WindowFn& fn) {
+    cudaStream_t st = ctx->stream;
+    const uint64_t W = ingest_window_bytes();
+    std::vector<uint64_t> cut{0};  // window w = [cut[w], cut[w + 1])
+    while (cut.back() < n_bytes) {
+        const uint64_t a = cut.back();
+        uint64_t b = n_bytes;
+        if (n_bytes - a > W) {
+            const uint64_t p = a + W - 1;
+            if (host_text) {
+                const void* q = memchr(host_text + p, '\n', n_bytes - p);
+                if (q) b = (uint64_t)((const char*)q - host_text) + 1;
+            } else {
+                char piece[4096];
+                for (uint64_t q = p; q < n_bytes && b == n_bytes; q += sizeof piece) {
+                    const uint64_t len = std::min<uint64_t>(sizeof piece, n_bytes - q);
+                    GT_CUDA(cudaMemcpyAsync(piece, dev_text + q, len, cudaMemcpyDeviceToHost, st));
+                    GT_CUDA(cudaStreamSynchronize(st));
+                    const void* nl = memchr(piece, '\n', len);
+                    if (nl) b = q + (uint64_t)((const char*)nl - piece) + 1;
+                }
+            }
+        }
+        if (b - a >= 0xFFFFFFF0ull) return fail(GTGPU_ERR_UNSUPPORTED, who + ": a line of 4 GiB or more");
+        cut.push_back(b);
+    }
+    const size_t n_win = cut.size() - 1;
+    uint64_t max_win = 0;
+    for (size_t w = 0; w < n_win; ++w) max_win = std::max(max_win, cut[w + 1] - cut[w]);
+    uint64_t first_line = 0;
+    uint32_t n_lines = 0;
+    if (dev_text) {
+        char* d_copy = nullptr;  // windows that do not start 16-byte aligned are moved to aligned scratch (the newline scan loads 16 B)
+        for (size_t w = 0; w < n_win; ++w) {
+            const char* d = dev_text + cut[w];
+            if (reinterpret_cast<uintptr_t>(d) & 15) {
+                if (!d_copy) GT_TRY(ctx->scratch_get(SC_WIN_A, max_win + 64, (void**)&d_copy));
+                GT_CUDA(cudaMemcpyAsync(d_copy, d, cut[w + 1] - cut[w], cudaMemcpyDeviceToDevice, st));
+                d = d_copy;
+            }
+            GT_TRY(fn(d, cut[w + 1] - cut[w], first_line, &n_lines));
+            first_line += n_lines;
+        }
+        return GTGPU_OK;
+    }
+    char* dbuf[2] = {nullptr, nullptr};
+    GT_TRY(ctx->scratch_get(SC_WIN_A, max_win + 64, (void**)&dbuf[0]));
+    if (n_win > 1) GT_TRY(ctx->scratch_get(SC_WIN_B, max_win + 64, (void**)&dbuf[1]));
+    StagingScope sg(ctx);
+    const uint64_t piece = std::min<uint64_t>(max_win, 64ull << 20);
+    for (int b = 0; b < 2; ++b) {
+        GT_TRY(ctx->pinned_get(piece, &sg.pin[b]));
+        GT_CUDA(cudaEventCreateWithFlags(&sg.ev[b], cudaEventDisableTiming));
+    }
+    // window w -> dbuf[w % 2] through the two pinned pieces; runs on a helper thread while the kernels of window w - 1 run
+    std::string stage_err;
+    auto stage = [&](size_t w) -> int32_t {
+        if (cudaSetDevice(ctx->device) != cudaSuccess) return GTGPU_ERR_CUDA;
+        cudaError_t e = cudaSuccess;
+        uint64_t j = 0;
+        for (uint64_t off = cut[w]; off < cut[w + 1] && e == cudaSuccess; off += piece, ++j) {
+            const int b = (int)(j & 1);
+            const uint64_t len = std::min(piece, cut[w + 1] - off);
+            if (sg.used[b]) e = cudaEventSynchronize(sg.ev[b]);
+            if (e != cudaSuccess) break;
+            memcpy(sg.pin[b].ptr, host_text + off, len);
+            e = cudaMemcpyAsync(dbuf[w & 1] + (off - cut[w]), sg.pin[b].ptr, len, cudaMemcpyHostToDevice, ctx->copy_in);
+            if (e == cudaSuccess) e = cudaEventRecord(sg.ev[b], ctx->copy_in);
+            sg.used[b] = true;
+        }
+        if (e == cudaSuccess) e = cudaStreamSynchronize(ctx->copy_in);
+        if (e != cudaSuccess) stage_err = std::string("H2D of the text: ") + cudaGetErrorString(e);
+        return e == cudaSuccess ? GTGPU_OK : GTGPU_ERR_CUDA;
+    };
+    int32_t s_next = stage(0);
+    for (size_t w = 0; w < n_win && s_next == GTGPU_OK; ++w) {
+        std::thread helper;
+        if (w + 1 < n_win) helper = std::thread([&, w] { s_next = stage(w + 1); });
+        const int32_t s = fn(dbuf[w & 1], cut[w + 1] - cut[w], first_line, &n_lines);
+        if (helper.joinable()) helper.join();
+        if (s != GTGPU_OK) return s;
+        first_line += n_lines;
+    }
+    if (s_next != GTGPU_OK) return fail(s_next, who + ": " + stage_err);
+    return GTGPU_OK;
+}
+
+static int32_t parse_error(const std::string& who, uint64_t line) {
+    return fail(GTGPU_ERR_INVALID, who + ": Failed to parse fragment at line " + std::to_string(line));
+}
+
+static int32_t too_many(const std::string& who) {
+    return fail(GTGPU_ERR_UNSUPPORTED, who + ": more than 2^32 - 1 fragments in one file");
+}
+
+// the caller holds ctx->mu
+static int32_t score_matrix_text_locked(gtgpu_index* ix, const char* host_text, const char* dev_text, uint64_t n_bytes,
+                                        uint32_t n_names, const char* names, const uint32_t* name_offsets, int32_t mode,
+                                        uint64_t n_cols, uint32_t* out_row, const std::string& who) {
+    gtgpu_ctx* ctx = ix->ctx;
+    cudaStream_t st = ctx->stream;
+    uint32_t* d_row;
+    GT_TRY(ctx->scratch_get(SC_MATRIX, std::max<uint64_t>(n_cols * 4, 4), (void**)&d_row));
+    GT_CUDA(cudaMemsetAsync(d_row, 0, n_cols * 4, st));
+    if (n_bytes) {
+        NameTable nt;
+        uint64_t* d_fo;
+        uint64_t total = 0;
+        GT_TRY(upload_name_table(ctx, n_names, names, name_offsets, &nt));
+        GT_TRY(ctx->scratch_get(SC_FILE_OFFS, 16, (void**)&d_fo));
+        GT_TRY(for_each_window(ctx, host_text, dev_text, n_bytes, who,
+                               [&](const char* d, uint64_t nb, uint64_t line0, uint32_t* n_lines) -> int32_t {
+            FragParse fp;
+            GT_TRY(parse_fragments_locked(ctx, d, nb, nt, FRAG_SCORE_MATRIX, &fp));
+            *n_lines = fp.n_lines;
+            if (fp.bad_line != 0xFFFFFFFFu) return parse_error(who, line0 + fp.bad_line);
+            total += fp.n;
+            if (total > 0xFFFFFFFFull) return too_many(who);
+            const uint64_t fo[2] = {0, fp.n};
+            GT_CUDA(cudaMemcpyAsync(d_fo, fo, 16, cudaMemcpyHostToDevice, st));
+            GT_TRY(score_matrix_dev_locked(ix, 1, d_fo, fp.n, fp.chr, fp.start, fp.end, mode, n_cols, d_row, true));
+            GT_CUDA(cudaStreamSynchronize(st));  // the window's buffers are reused by the next one
+            return GTGPU_OK;
+        }));
+    }
+    if (n_cols) GT_CUDA(cudaMemcpyAsync(out_row, d_row, n_cols * 4, cudaMemcpyDeviceToHost, st));
+    GT_CUDA(cudaStreamSynchronize(st));
+    return GTGPU_OK;
+}
+
+// the caller holds ctx->mu
+static int32_t score_barcodes_text_locked(gtgpu_index* ix, const char* host_text, const char* dev_text, uint64_t n_bytes,
+                                          uint32_t n_names, const char* names, const uint32_t* name_offsets, uint32_t* out_n_barcodes,
+                                          gtgpu_buf** out_names, gtgpu_buf** out_name_offsets, gtgpu_buf** out_barcode_offsets,
+                                          gtgpu_buf** out_peaks, gtgpu_buf** out_counts, const std::string& who) {
+    gtgpu_ctx* ctx = ix->ctx;
+    FragBarcodeTable tab;
+    if (n_bytes) {
+        NameTable nt;
+        GT_TRY(upload_name_table(ctx, n_names, names, name_offsets, &nt));
+        GT_TRY(for_each_window(ctx, host_text, dev_text, n_bytes, who,
+                               [&](const char* d, uint64_t nb, uint64_t line0, uint32_t* n_lines) -> int32_t {
+            FragParse fp;
+            GT_TRY(parse_fragments_locked(ctx, d, nb, nt, FRAG_SCORE_BARCODES, &fp));
+            *n_lines = fp.n_lines;
+            if (fp.bad_line != 0xFFFFFFFFu) return parse_error(who, line0 + fp.bad_line);
+            if (tab.n + fp.n > 0xFFFFFFFFull) return too_many(who);
+            return tab.add_window(ctx, d, fp, n_names);
+        }));
+    }
+    uint32_t n_kept = 0;
+    gtgpu_buf *nm = nullptr, *no = nullptr;
+    GT_TRY(tab.finish(ctx, &n_kept, &nm, &no));
+    gtgpu_buf* offs = new gtgpu_buf();
+    offs->ctx = ctx;
+    offs->len = (uint64_t)n_kept + 1;
+    offs->elem_size = 8;
+    int32_t s = ctx->pinned_get(offs->len * 8, &offs->block);
+    if (s == GTGPU_OK)
+        s = score_barcodes_dev_locked(ix, tab.n, tab.chr.u32(), tab.start.u32(), tab.end.u32(), tab.bc.u32(), n_kept,
+                                      (uint64_t*)offs->block.ptr, out_peaks, out_counts);
+    if (s != GTGPU_OK) {
+        for (gtgpu_buf* b : {nm, no, offs}) {
+            if (b->block.ptr) ctx->pinned_put(b->block);
+            delete b;
+        }
+        return s;
+    }
+    *out_n_barcodes = n_kept;
+    *out_names = nm;
+    *out_name_offsets = no;
+    *out_barcode_offsets = offs;
+    return GTGPU_OK;
+}
+
+// gzip members -> device text (SC_GZ_OUT); a text that does not fit in device memory is reported as such
+static int32_t inflate_for_scoring(gtgpu_ctx* ctx, uint64_t n_members, const uint8_t* gz, const uint64_t* member_offsets,
+                                   const std::string& who, uint8_t** d_text, uint64_t* n_text) {
+    const int32_t s = gunzip_locked(ctx, n_members, gz, member_offsets, nullptr, d_text, n_text);
+    if (s == GTGPU_ERR_NOMEM)
+        return fail(s, who + ": the inflated text does not fit in device memory (gzip input is inflated whole before it is parsed): " +
+                           gtgpu_last_error());
+    return s;
+}
+
+}  // namespace gtgpu
+
+extern "C" int32_t gtgpu_score_matrix_text(gtgpu_index* ix, const char* text, uint64_t n_bytes, uint32_t n_names, const char* names,
+                                           const uint32_t* name_offsets, int32_t mode, uint64_t n_cols, uint32_t* out_row) try {
+    if (!ix || (n_cols && !out_row) || (n_bytes && !text) || (n_names && (!names || !name_offsets)))
+        return fail(GTGPU_ERR_INVALID, "score_matrix_text: null argument");
+    if (mode != GTGPU_SCORE_ATAC && mode != GTGPU_SCORE_CHIP) return fail(GTGPU_ERR_INVALID, "score_matrix_text: unknown mode");
+    gtgpu_ctx* ctx = ix->ctx;
+    std::lock_guard<std::mutex> lk(ctx->mu);
+    GT_CUDA(cudaSetDevice(ctx->device));
+    return score_matrix_text_locked(ix, text, nullptr, n_bytes, n_names, names, name_offsets, mode, n_cols, out_row, "score_matrix_text");
+} GT_CATCH
+
+extern "C" int32_t gtgpu_score_matrix_gz(gtgpu_index* ix, uint64_t n_members, const uint8_t* gz, const uint64_t* member_offsets,
+                                         uint32_t n_names, const char* names, const uint32_t* name_offsets, int32_t mode, uint64_t n_cols,
+                                         uint32_t* out_row) try {
+    if (!ix || (n_cols && !out_row) || (n_names && (!names || !name_offsets))) return fail(GTGPU_ERR_INVALID, "score_matrix_gz: null argument");
+    if (mode != GTGPU_SCORE_ATAC && mode != GTGPU_SCORE_CHIP) return fail(GTGPU_ERR_INVALID, "score_matrix_gz: unknown mode");
+    GT_TRY(check_members(n_members, gz, member_offsets, "score_matrix_gz"));
+    gtgpu_ctx* ctx = ix->ctx;
+    std::lock_guard<std::mutex> lk(ctx->mu);
+    GT_CUDA(cudaSetDevice(ctx->device));
+    uint8_t* d_text = nullptr;
+    uint64_t n_text = 0;
+    GT_TRY(inflate_for_scoring(ctx, n_members, gz, member_offsets, "score_matrix_gz", &d_text, &n_text));
+    return score_matrix_text_locked(ix, nullptr, (const char*)d_text, n_text, n_names, names, name_offsets, mode, n_cols, out_row,
+                                    "score_matrix_gz");
+} GT_CATCH
+
+extern "C" int32_t gtgpu_score_barcodes_text(gtgpu_index* ix, const char* text, uint64_t n_bytes, uint32_t n_names, const char* names,
+                                             const uint32_t* name_offsets, uint32_t* out_n_barcodes, gtgpu_buf** out_barcode_names,
+                                             gtgpu_buf** out_barcode_name_offsets, gtgpu_buf** out_barcode_offsets,
+                                             gtgpu_buf** out_peaks, gtgpu_buf** out_counts) try {
+    if (!ix || !out_n_barcodes || !out_barcode_names || !out_barcode_name_offsets || !out_barcode_offsets || !out_peaks || !out_counts ||
+        (n_bytes && !text) || (n_names && (!names || !name_offsets)))
+        return fail(GTGPU_ERR_INVALID, "score_barcodes_text: null argument");
+    gtgpu_ctx* ctx = ix->ctx;
+    std::lock_guard<std::mutex> lk(ctx->mu);
+    GT_CUDA(cudaSetDevice(ctx->device));
+    return score_barcodes_text_locked(ix, text, nullptr, n_bytes, n_names, names, name_offsets, out_n_barcodes, out_barcode_names,
+                                      out_barcode_name_offsets, out_barcode_offsets, out_peaks, out_counts, "score_barcodes_text");
+} GT_CATCH
+
+extern "C" int32_t gtgpu_score_barcodes_gz(gtgpu_index* ix, uint64_t n_members, const uint8_t* gz, const uint64_t* member_offsets,
+                                           uint32_t n_names, const char* names, const uint32_t* name_offsets, uint32_t* out_n_barcodes,
+                                           gtgpu_buf** out_barcode_names, gtgpu_buf** out_barcode_name_offsets,
+                                           gtgpu_buf** out_barcode_offsets, gtgpu_buf** out_peaks, gtgpu_buf** out_counts) try {
+    if (!ix || !out_n_barcodes || !out_barcode_names || !out_barcode_name_offsets || !out_barcode_offsets || !out_peaks || !out_counts ||
+        (n_names && (!names || !name_offsets)))
+        return fail(GTGPU_ERR_INVALID, "score_barcodes_gz: null argument");
+    GT_TRY(check_members(n_members, gz, member_offsets, "score_barcodes_gz"));
+    gtgpu_ctx* ctx = ix->ctx;
+    std::lock_guard<std::mutex> lk(ctx->mu);
+    GT_CUDA(cudaSetDevice(ctx->device));
+    uint8_t* d_text = nullptr;
+    uint64_t n_text = 0;
+    GT_TRY(inflate_for_scoring(ctx, n_members, gz, member_offsets, "score_barcodes_gz", &d_text, &n_text));
+    return score_barcodes_text_locked(ix, nullptr, (const char*)d_text, n_text, n_names, names, name_offsets, out_n_barcodes,
+                                      out_barcode_names, out_barcode_name_offsets, out_barcode_offsets, out_peaks, out_counts,
+                                      "score_barcodes_gz");
 } GT_CATCH

@@ -884,6 +884,75 @@ std::vector<std::pair<std::string, std::map<uint32_t, uint32_t>>> barcode_scorin
     return out;
 }
 
+// Device parse of one fragment file: a bgzip'ed file goes to the device inflater (gz_members_for_device), any other file is
+// read by read_file_bytes (a single-member gzip is inflated by zlib on the host).  Device errors are prefixed with the path.
+namespace {
+struct FragmentBytes {
+    std::string raw, text;
+    std::vector<uint64_t> members;
+    bool gz = false;
+    explicit FragmentBytes(const std::string& path) {
+        gz = gz_members_for_device(path, raw, members);
+        if (!gz) text = read_file_bytes(path);
+    }
+};
+void check_file(int32_t status, const std::string& path) {
+    if (status != GTGPU_OK) throw Error(path + ": " + gtgpu_last_error());
+}
+}  // namespace
+
+CountMatrix region_scoring_from_fragments_device(const std::vector<std::string>& fragment_files, const ConsensusSet& consensus,
+                                                 ScoringMode mode) {
+    NameBlob nb(consensus.chroms());
+    CountMatrix m;
+    m.rows = fragment_files.size();
+    m.cols = consensus.len();
+    m.data.assign(m.rows * m.cols, 0);
+    for (size_t f = 0; f < fragment_files.size(); ++f) {
+        const std::string& path = fragment_files[f];
+        FragmentBytes fb(path);
+        uint32_t* row = m.data.data() + f * m.cols;
+        if (fb.gz)
+            check_file(gtgpu_score_matrix_gz(consensus.index(), fb.members.size() - 1, (const uint8_t*)fb.raw.data(), fb.members.data(),
+                                             (uint32_t)consensus.chroms().size(), nb.blob.data(), nb.offsets.data(), (int32_t)mode, m.cols, row),
+                       path);
+        else
+            check_file(gtgpu_score_matrix_text(consensus.index(), fb.text.data(), fb.text.size(), (uint32_t)consensus.chroms().size(),
+                                               nb.blob.data(), nb.offsets.data(), (int32_t)mode, m.cols, row),
+                       path);
+    }
+    return m;
+}
+
+std::vector<std::pair<std::string, std::map<uint32_t, uint32_t>>> barcode_scoring_from_fragments_device(const std::string& fragment_file,
+                                                                                                        const ConsensusSet& consensus) {
+    NameBlob nb(consensus.chroms());
+    FragmentBytes fb(fragment_file);
+    uint32_t n_barcodes = 0;
+    PinnedResult names, name_offsets, offsets, peaks, counts;
+    if (fb.gz)
+        check_file(gtgpu_score_barcodes_gz(consensus.index(), fb.members.size() - 1, (const uint8_t*)fb.raw.data(), fb.members.data(),
+                                           (uint32_t)consensus.chroms().size(), nb.blob.data(), nb.offsets.data(), &n_barcodes, &names.buf,
+                                           &name_offsets.buf, &offsets.buf, &peaks.buf, &counts.buf),
+                   fragment_file);
+    else
+        check_file(gtgpu_score_barcodes_text(consensus.index(), fb.text.data(), fb.text.size(), (uint32_t)consensus.chroms().size(),
+                                             nb.blob.data(), nb.offsets.data(), &n_barcodes, &names.buf, &name_offsets.buf, &offsets.buf,
+                                             &peaks.buf, &counts.buf),
+                   fragment_file);
+    const char* blob = (const char*)gtgpu_buf_data(names.buf);
+    const uint64_t* noff = (const uint64_t*)gtgpu_buf_data(name_offsets.buf);
+    const uint64_t* off = (const uint64_t*)gtgpu_buf_data(offsets.buf);
+    std::vector<std::pair<std::string, std::map<uint32_t, uint32_t>>> out;
+    out.reserve(n_barcodes);
+    for (uint32_t b = 0; b < n_barcodes; ++b) {
+        std::map<uint32_t, uint32_t> m;
+        for (uint64_t k = off[b]; k < off[b + 1]; ++k) m[peaks.data()[k]] = counts.data()[k];
+        out.emplace_back(std::string(blob + noff[b], noff[b + 1] - noff[b]), std::move(m));
+    }
+    return out;
+}
+
 // ---- Igd / LOLA -----------------------------------------------------------------------------------------------------------------
 Igd::Igd(std::shared_ptr<Device> dev, const std::vector<const RegionSet*>& sets) : dev_(std::move(dev)), n_files_(sets.size()) {
     std::vector<uint64_t> file_offsets(sets.size() + 1, 0);

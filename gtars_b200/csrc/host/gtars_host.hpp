@@ -173,6 +173,13 @@ CountMatrix region_scoring_from_fragments(const std::vector<std::string>& fragme
 std::vector<std::pair<std::string, std::map<uint32_t, uint32_t>>> barcode_scoring_from_fragments(const std::string& fragment_file,
                                                                                                  const ConsensusSet& consensus);
 
+// The same two with every file's bytes parsed on the device (gtgpu_score_matrix_text / gtgpu_score_barcodes_text, or their
+// _gz forms for bgzip'ed files), one call per file; results and errors as above (an error names the file).
+CountMatrix region_scoring_from_fragments_device(const std::vector<std::string>& fragment_files, const ConsensusSet& consensus,
+                                                 ScoringMode mode);
+std::vector<std::pair<std::string, std::map<uint32_t, uint32_t>>> barcode_scoring_from_fragments_device(const std::string& fragment_file,
+                                                                                                        const ConsensusSet& consensus);
+
 // ---- gtars_tokenizers ----------------------------------------------------------------------------------------------------
 struct SpecialTokens {
     std::string unk = "<unk>", pad = "<pad>", mask = "<mask>", cls = "<cls>", eos = "<eos>", bos = "<bos>", sep = "<sep>";

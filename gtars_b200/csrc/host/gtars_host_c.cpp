@@ -234,6 +234,26 @@ void* gth_tokenizer_fragments_device(void* t, const char* path) {
         return l;
     }, nullptr);
 }
+int gth_region_scoring_device(void* c, uint64_t n_files, const char** paths, int mode, uint32_t* out /* n_files x len */) {
+    return guard([&]() -> int {
+        std::vector<std::string> files(paths, paths + n_files);
+        CountMatrix m = region_scoring_from_fragments_device(files, *(ConsensusSet*)c, (ScoringMode)mode);
+        std::copy(m.data.begin(), m.data.end(), out);
+        return 0;
+    }, 1);
+}
+void* gth_barcode_scoring_device(void* c, const char* path) {
+    return guard([&]() -> void* {
+        Lists* l = new Lists();
+        for (auto& kv : barcode_scoring_from_fragments_device(path, *(ConsensusSet*)c)) {
+            l->names.push_back(kv.first);
+            std::vector<uint32_t> flat;
+            for (auto& pc : kv.second) { flat.push_back(pc.first); flat.push_back(pc.second); }
+            l->lists.push_back(std::move(flat));
+        }
+        return l;
+    }, nullptr);
+}
 void* gth_tokenizer_fragments(void* t, const char* path) {
     return guard([&]() -> void* {
         Lists* l = new Lists();

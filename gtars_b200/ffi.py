@@ -63,6 +63,10 @@ SIGNATURES = {
     "gtgpu_score_matrix": (_i32, [_vp, _u64, _vp, _u64, _vp, _vp, _vp, _i32, _u64, _vp]),
     "gtgpu_score_matrix_dev": (_i32, [_vp, _u64, _vp, _u64, _vp, _vp, _vp, _i32, _u64, _vp]),
     "gtgpu_score_barcodes": (_i32, [_vp, _u64, _vp, _vp, _vp, _vp, _u32, _vp, _vp, _vp]),
+    "gtgpu_score_matrix_text": (_i32, [_vp, _vp, _u64, _u32, _vp, _vp, _i32, _u64, _vp]),
+    "gtgpu_score_matrix_gz": (_i32, [_vp, _u64, _vp, _vp, _u32, _vp, _vp, _i32, _u64, _vp]),
+    "gtgpu_score_barcodes_text": (_i32, [_vp, _vp, _u64, _u32, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp]),
+    "gtgpu_score_barcodes_gz": (_i32, [_vp, _u64, _vp, _vp, _u32, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp]),
     "gtgpu_igd_build": (_i32, [_vp, _u64, _vp, _u32, _vp, _vp, _vp, _vp]),
     "gtgpu_igd_free": (_i32, [_vp]),
     "gtgpu_igd_info": (_i32, [_vp, _vp]),
@@ -390,6 +394,35 @@ class Index:
                                          _p(out_off), C.byref(hp), C.byref(hc)))
         return out_off, _take(hp), _take(hc)
 
+    def score_matrix_text(self, text: bytes, chrom_names, mode, n_cols, gz_member_offsets=None):
+        """gtgpu_score_matrix_text (or _gz when gz_member_offsets is given: `text` is then the gzip data): the file's
+        uint32 row [n_cols] of region_scoring_from_fragments, parsed on the device."""
+        blob, offs = _names_blob(chrom_names)
+        out = np.empty(n_cols, dtype=np.uint32)
+        if gz_member_offsets is not None:
+            mo = _arr(gz_member_offsets, np.uint64)
+            check(lib().gtgpu_score_matrix_gz(self._h, len(mo) - 1, text, _p(mo), len(chrom_names), blob, _p(offs), mode, n_cols,
+                                              _p(out)))
+        else:
+            check(lib().gtgpu_score_matrix_text(self._h, _text_ptr(text), _text_len(text), len(chrom_names), blob, _p(offs), mode, n_cols,
+                                                _p(out)))
+        return out
+
+    def score_barcodes_text(self, text: bytes, chrom_names, gz_member_offsets=None):
+        """gtgpu_score_barcodes_text (or _gz): ([barcode strings], offsets[n + 1], peaks, counts) sorted by (barcode, peak)."""
+        blob, offs = _names_blob(chrom_names)
+        nb = C.c_uint32(0)
+        hn, hno, ho, hp, hc = C.c_void_p(), C.c_void_p(), C.c_void_p(), C.c_void_p(), C.c_void_p()
+        outs = (C.byref(nb), C.byref(hn), C.byref(hno), C.byref(ho), C.byref(hp), C.byref(hc))
+        if gz_member_offsets is not None:
+            mo = _arr(gz_member_offsets, np.uint64)
+            check(lib().gtgpu_score_barcodes_gz(self._h, len(mo) - 1, text, _p(mo), len(chrom_names), blob, _p(offs), *outs))
+        else:
+            check(lib().gtgpu_score_barcodes_text(self._h, _text_ptr(text), _text_len(text), len(chrom_names), blob, _p(offs), *outs))
+        names = _take(hn, dtype=np.uint8).tobytes()
+        no = _take(hno, dtype=np.uint64)
+        return ([names[int(a):int(b)].decode() for a, b in zip(no[:-1], no[1:])], _take(ho, dtype=np.uint64), _take(hp), _take(hc))
+
     # ---- device-resident entry points (raw device pointers as ints) ----------------------------------------------------
     def count_dev(self, n, d_chr, d_start, d_end, min_overlap, d_out):
         check(lib().gtgpu_count_dev(self._h, n, d_chr, d_start, d_end, min_overlap, d_out))
@@ -468,6 +501,15 @@ def gunzip(ctx: "Context", gz: bytes, member_offsets=None):
     h = C.c_void_p()
     check(lib().gtgpu_gunzip(ctx._h, len(mo) - 1, gz, _p(mo), C.byref(h), _p(out_off)))
     return _take(h, dtype=np.uint8).tobytes(), out_off
+
+
+def _text_ptr(text):
+    """bytes, or a uint8 numpy array (a multi-GB text need not be copied into a bytes object)"""
+    return _p(text) if isinstance(text, np.ndarray) else text
+
+
+def _text_len(text):
+    return text.nbytes if isinstance(text, np.ndarray) else len(text)
 
 
 def _names_blob(chrom_names):

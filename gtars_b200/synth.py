@@ -177,3 +177,45 @@ def group_by_chrom(chr_: torch.Tensor, start: torch.Tensor, end: torch.Tensor) -
     offs = torch.zeros(N_CHROMS + 1, dtype=torch.int64, device=chr_.device)
     offs[1:] = torch.cumsum(counts, 0)
     return dict(chrom_offsets=offs, g_start=start[grp], g_end=end[grp], g_val=grp.int())
+
+
+# ---- fragment files as text (numpy, for the text-ingest paths) ------------------------------------------------------------------
+FRAGMENT_LINE = 40  # "chrNN" padded to 5 + TAB + 10-digit start + TAB + 10-digit end + TAB + "BC" + 7 digits + TAB + "1" + LF
+
+
+def make_fragment_arrays(n: int, seed: int, n_barcodes: int):
+    """Seeded fragments on the hg38-shaped chromosomes: (chr id into CHROM_NAMES, start, end, barcode number) as numpy
+    uint32 arrays, 40 .. 1000 bp long."""
+    import numpy as np
+    rng = np.random.default_rng(seed)
+    sizes = np.array(CHROM_SIZES, dtype=np.int64)
+    c = rng.choice(len(sizes), n, p=sizes / sizes.sum()).astype(np.uint32)
+    s = (rng.random(n) * (sizes[c] - 2000)).astype(np.uint32)
+    e = s + rng.integers(40, 1000, n, dtype=np.uint32)
+    b = rng.integers(0, n_barcodes, n, dtype=np.uint32)
+    return c, s, e, b
+
+
+def fragment_text(chr_id, start, end, barcode):
+    """Vectorised fixed-width fragment lines as a uint8 array (FRAGMENT_LINE bytes each): the name padded with spaces (split
+    on whitespace like any separator), start / end zero-padded (str::parse::<u32> accepts leading zeros), barcode "BC%07d",
+    support 1.  barcode < 10^7."""
+    import numpy as np
+    tab = np.array([list(nm.ljust(5).encode()) for nm in CHROM_NAMES], dtype=np.uint8)
+    out = np.empty((len(start), FRAGMENT_LINE), dtype=np.uint8)
+    out[:, 0:5] = tab[chr_id]
+    out[:, [5, 16, 27, 37]] = 9
+
+    def digits(col, v, width):
+        v = np.asarray(v).astype(np.uint64)
+        for j in range(width - 1, -1, -1):
+            out[:, col + j] = (v % 10).astype(np.uint8) + 48
+            v //= 10
+
+    digits(6, start, 10)
+    digits(17, end, 10)
+    out[:, 28:30] = np.frombuffer(b"BC", dtype=np.uint8)
+    digits(30, barcode, 7)
+    out[:, 38] = ord("1")
+    out[:, 39] = 10
+    return out.reshape(-1)

@@ -283,6 +283,35 @@ int32_t gtgpu_score_matrix_dev(gtgpu_index* index, uint64_t n_files, const uint6
                                const uint32_t* d_chr, const uint32_t* d_start, const uint32_t* d_end, int32_t mode,
                                uint64_t n_cols, uint32_t* d_out_counts);
 
+/* region_scoring_from_fragments / barcode_scoring_from_fragments from ONE fragment file's bytes, parsed on the device: the
+ * (decompressed) text, or its gzip members (n_members, gz, member_offsets as in gtgpu_gunzip; inflated whole into device memory,
+ * GTGPU_ERR_NOMEM when that text does not fit).  Lines follow Fragment::from_str (gtars-core/src/models/fragments.rs:16-44):
+ * '#' lines are skipped, every other line needs at least five whitespace-separated fields with start, end and the fifth
+ * (support) field accepted by str::parse::<u32>() — otherwise GTGPU_ERR_INVALID, "Failed to parse fragment at line i" with the
+ * 0-based line index the host parser reports ('#' lines count), and no output.  Chromosome names map through the caller's table
+ * as in gtgpu_tokenize_fragments_text.  Any file size: the text is parsed in windows of about GTGPU_INGEST_WINDOW bytes (default
+ * 2 GiB); at most 2^32 - 1 fragments per file (GTGPU_ERR_UNSUPPORTED beyond).
+ * gtgpu_score_matrix_text / _gz: out_row (n_cols u32, overwritten) = the file's row of gtgpu_score_matrix, same mode and n_cols
+ * rules.  gtgpu_score_barcodes_text / _gz: the content of gtgpu_score_barcodes for the file, barcodes numbered in
+ * first-appearance order; only barcodes with at least one fragment on a chromosome of the name table are kept (the reference's
+ * key set, files.rs:106-129 + fragment_scoring.rs:146-153: such a barcode has an entry even without a hit).  Outputs:
+ * *out_n_barcodes (kept barcodes); *out_barcode_names = their bytes back to back in id order (u8 elements);
+ * *out_barcode_name_offsets = n_barcodes + 1 u64 offsets into those bytes; *out_barcode_offsets = n_barcodes + 1 u64 offsets into
+ * *out_peaks / *out_counts (u32 each), sorted by (barcode, peak).  On a multi-device ctx these run on the first device. */
+int32_t gtgpu_score_matrix_text(gtgpu_index* index, const char* text, uint64_t n_bytes, uint32_t n_names, const char* names,
+                                const uint32_t* name_offsets, int32_t mode, uint64_t n_cols, uint32_t* out_row);
+int32_t gtgpu_score_matrix_gz(gtgpu_index* index, uint64_t n_members, const uint8_t* gz, const uint64_t* member_offsets,
+                              uint32_t n_names, const char* names, const uint32_t* name_offsets, int32_t mode, uint64_t n_cols,
+                              uint32_t* out_row);
+int32_t gtgpu_score_barcodes_text(gtgpu_index* index, const char* text, uint64_t n_bytes, uint32_t n_names, const char* names,
+                                  const uint32_t* name_offsets, uint32_t* out_n_barcodes, gtgpu_buf** out_barcode_names,
+                                  gtgpu_buf** out_barcode_name_offsets, gtgpu_buf** out_barcode_offsets, gtgpu_buf** out_peaks,
+                                  gtgpu_buf** out_counts);
+int32_t gtgpu_score_barcodes_gz(gtgpu_index* index, uint64_t n_members, const uint8_t* gz, const uint64_t* member_offsets,
+                                uint32_t n_names, const char* names, const uint32_t* name_offsets, uint32_t* out_n_barcodes,
+                                gtgpu_buf** out_barcode_names, gtgpu_buf** out_barcode_name_offsets, gtgpu_buf** out_barcode_offsets,
+                                gtgpu_buf** out_peaks, gtgpu_buf** out_counts);
+
 /* barcode_scoring_from_fragments (fragment_scoring.rs:126-155): whole fragments, sparse barcode x peak counts.  The
  * reference returns HashMap<barcode, HashMap<peak, count>>; here the same content as CSR sorted by (barcode, peak):
  * out_barcode_offsets[n_barcodes + 1] index the (peak, count) pairs in *out_peaks / *out_counts. */
