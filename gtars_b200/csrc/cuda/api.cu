@@ -98,6 +98,7 @@ int32_t gtgpu_ctx::scratch_get(int role, size_t bytes, void** out) {
 
 int32_t gtgpu_ctx::pinned_get(size_t bytes, PinnedBlock* out) {
     bytes = std::max<size_t>(bytes, 64);
+    std::lock_guard<std::mutex> lk(pinned_mu);
     int best = -1;
     for (size_t i = 0; i < pinned_free.size(); ++i)
         if (pinned_free[i].cap >= bytes && (best < 0 || pinned_free[i].cap < pinned_free[best].cap)) best = (int)i;
@@ -123,6 +124,7 @@ int32_t gtgpu_ctx::pinned_get(size_t bytes, PinnedBlock* out) {
 
 void gtgpu_ctx::pinned_put(PinnedBlock b) {
     if (!b.ptr) return;
+    std::lock_guard<std::mutex> lk(pinned_mu);
     pinned_free.push_back(b);
     // keep at most 8 blocks; drop the smallest first
     while (pinned_free.size() > 8) {
@@ -132,6 +134,26 @@ void gtgpu_ctx::pinned_put(PinnedBlock b) {
         cudaFreeHost(pinned_free[k].ptr);
         pinned_free.erase(pinned_free.begin() + k);
     }
+}
+
+int32_t gtgpu::buf_new(gtgpu_ctx* ctx, uint64_t len, uint32_t elem_size, BufPtr* out) {
+    BufPtr buf(new (std::nothrow) gtgpu_buf());
+    if (!buf) return fail(GTGPU_ERR_NOMEM, "out of host memory (result buffer)");
+    buf->ctx = ctx;
+    buf->len = len;
+    buf->elem_size = elem_size;
+    GT_TRY(ctx->pinned_get(len * elem_size, &buf->block));
+    *out = std::move(buf);
+    return GTGPU_OK;
+}
+
+int32_t gtgpu::buf_from_device(gtgpu_ctx* ctx, const void* d_src, uint64_t len, uint32_t elem_size, cudaStream_t st, BufPtr* out) {
+    BufPtr buf;
+    GT_TRY(buf_new(ctx, len, elem_size, &buf));
+    const cudaError_t e = len ? cudaMemcpyAsync(buf->block.ptr, d_src, len * elem_size, cudaMemcpyDeviceToHost, st) : cudaSuccess;
+    if (e != cudaSuccess) return fail(GTGPU_ERR_CUDA, cudaGetErrorString(e));
+    *out = std::move(buf);
+    return GTGPU_OK;
 }
 
 void gtgpu_ctx::time_begin() {
@@ -314,10 +336,7 @@ const void* gtgpu_buf_data(const gtgpu_buf* buf) { return buf ? buf->block.ptr :
 uint64_t gtgpu_buf_len(const gtgpu_buf* buf) { return buf ? buf->len : 0; }
 int32_t gtgpu_buf_free(gtgpu_buf* buf) try {
     if (!buf) return GTGPU_OK;
-    {
-        std::lock_guard<std::mutex> lk(buf->ctx->mu);
-        buf->ctx->pinned_put(buf->block);
-    }
+    buf->ctx->pinned_put(buf->block);
     delete buf;
     return GTGPU_OK;
 } GT_CATCH
@@ -366,7 +385,7 @@ int32_t count_host(gtgpu_index* ix, uint64_t n, const uint32_t* chr, const uint3
 // Shared body of gtgpu_find (per-query offsets, no files) and gtgpu_tokenize_files (per-file offsets + [unk]).
 int32_t find_host(gtgpu_index* ix, uint64_t n, const uint32_t* chr, const uint32_t* start, const uint32_t* end,
                   int32_t min_overlap, uint64_t* out_offsets, bool files, uint64_t n_files,
-                  const uint64_t* file_offsets, uint32_t unk_id, uint64_t* out_file_tok, gtgpu_buf** out_ids) {
+                  const uint64_t* file_offsets, uint32_t unk_id, uint64_t* out_file_tok, BufPtr* out_ids) {
     gtgpu_ctx* ctx = ix->ctx;
     std::lock_guard<std::mutex> lk(ctx->mu);
     GT_CUDA(cudaSetDevice(ctx->device));
@@ -418,27 +437,19 @@ int32_t find_host(gtgpu_index* ix, uint64_t n, const uint32_t* chr, const uint32
         d_final = d_ids2;
     }
 
-    gtgpu_buf* buf = new gtgpu_buf();
-    buf->ctx = ctx;
-    buf->len = final_total;
-    int32_t s = ctx->pinned_get(final_total * 4, &buf->block);
-    if (s != GTGPU_OK) {
-        delete buf;
-        return s;
-    }
+    BufPtr buf;
+    const int32_t s = buf_from_device(ctx, d_final, final_total, 4, st, &buf);
+    if (s == GTGPU_ERR_CUDA) return fail(s, std::string("find: D2H: ") + gtgpu_last_error());
+    GT_TRY(s);
     cudaError_t e = cudaSuccess;
-    if (final_total) e = cudaMemcpyAsync(buf->block.ptr, d_final, final_total * 4, cudaMemcpyDeviceToHost, st);
-    if (e == cudaSuccess && files)
-        e = cudaMemcpyAsync(out_file_tok, d_out_tok, (n_files + 1) * 8, cudaMemcpyDeviceToHost, st);
-    if (e == cudaSuccess && !files)
-        e = cudaMemcpyAsync(out_offsets, d_offsets, (n + 1) * 8, cudaMemcpyDeviceToHost, st);
+    if (files) e = cudaMemcpyAsync(out_file_tok, d_out_tok, (n_files + 1) * 8, cudaMemcpyDeviceToHost, st);
+    else e = cudaMemcpyAsync(out_offsets, d_offsets, (n + 1) * 8, cudaMemcpyDeviceToHost, st);
     if (e == cudaSuccess) e = cudaStreamSynchronize(st);
     if (e != cudaSuccess) {
-        ctx->pinned_put(buf->block);
-        delete buf;
+        cudaStreamSynchronize(st);  // the ids' copy may still run
         return fail(GTGPU_ERR_CUDA, std::string("find: D2H: ") + cudaGetErrorString(e));
     }
-    *out_ids = buf;
+    *out_ids = std::move(buf);
     return GTGPU_OK;
 }
 
@@ -459,44 +470,27 @@ int32_t count_group(gtgpu_index* ix, uint64_t n, const uint32_t* chr, const uint
 }
 
 // Concatenates per-shard results (library-owned pinned buffers) into one buffer of the group's first device.
-int32_t merge_bufs(gtgpu_ctx* ctx0, std::vector<gtgpu_buf*>& parts, gtgpu_buf** out) {
+int32_t merge_bufs(gtgpu_ctx* ctx0, const std::vector<BufPtr>& parts, gtgpu_buf** out) {
     uint64_t total = 0;
-    for (auto* p : parts) total += p ? p->len : 0;
-    gtgpu_buf* buf = new gtgpu_buf();
-    buf->ctx = ctx0;
-    buf->len = total;
-    int32_t s;
-    {
-        std::lock_guard<std::mutex> lk(ctx0->mu);
-        cudaSetDevice(ctx0->device);
-        s = ctx0->pinned_get(total * 4, &buf->block);
-    }
-    if (s != GTGPU_OK) {
-        delete buf;
-        return s;
-    }
+    for (auto& p : parts) total += p ? p->len : 0;
+    cudaSetDevice(ctx0->device);
+    BufPtr buf;
+    GT_TRY(buf_new(ctx0, total, 4, &buf));
     std::vector<uint64_t> base(parts.size() + 1, 0);
     for (size_t r = 0; r < parts.size(); ++r) base[r + 1] = base[r] + (parts[r] ? parts[r]->len : 0);
     for_each_device(parts.size(), [&](size_t r) -> int32_t {
         if (parts[r] && parts[r]->len) memcpy((uint32_t*)buf->block.ptr + base[r], parts[r]->block.ptr, parts[r]->len * 4);
         return GTGPU_OK;
     });
-    *out = buf;
+    *out = buf.release();
     return GTGPU_OK;
-}
-
-void free_parts(std::vector<gtgpu_buf*>& parts) {
-    for (auto*& p : parts) {
-        if (p) gtgpu_buf_free(p);
-        p = nullptr;
-    }
 }
 
 int32_t find_group(gtgpu_index* ix, uint64_t n, const uint32_t* chr, const uint32_t* start, const uint32_t* end, int32_t min_overlap,
                    uint64_t* out_offsets, gtgpu_buf** out_vals) {
     std::lock_guard<std::mutex> glk(ix->ctx->group_mu);
     const size_t D = ix->replicas.size();
-    std::vector<gtgpu_buf*> parts(D, nullptr);
+    std::vector<BufPtr> parts(D);
     std::vector<std::vector<uint64_t>> offs(D);
     int32_t s = for_each_device(D, [&](size_t r) -> int32_t {
         uint64_t lo, hi;
@@ -516,7 +510,6 @@ int32_t find_group(gtgpu_index* ix, uint64_t n, const uint32_t* chr, const uint3
         }
         out_offsets[n] = base;
     }
-    free_parts(parts);
     return s;
 }
 
@@ -526,7 +519,7 @@ int32_t tokenize_files_group_simple(gtgpu_index* ix, uint64_t n_files, const uin
                                     const uint32_t* start, const uint32_t* end, uint32_t unk_id, uint64_t* out_file_tok,
                                     gtgpu_buf** out_ids) {
     const size_t D = ix->replicas.size();
-    std::vector<gtgpu_buf*> parts(D, nullptr);
+    std::vector<BufPtr> parts(D);
     std::vector<std::vector<uint64_t>> fo(D), tok(D);
     int32_t s = for_each_device(D, [&](size_t r) -> int32_t {
         uint64_t f0, f1;
@@ -549,7 +542,6 @@ int32_t tokenize_files_group_simple(gtgpu_index* ix, uint64_t n_files, const uin
         }
         out_file_tok[n_files] = base;
     }
-    free_parts(parts);
     return s;
 }
 
@@ -558,7 +550,10 @@ int32_t tokenize_files_plain(gtgpu_index* ix, uint64_t n, uint64_t n_files, cons
                              const uint32_t* start, const uint32_t* end, uint32_t unk_id, uint64_t* out_file_tok, gtgpu_buf** out_ids) {
     if (is_group(ix) && n >= (1u << 20) && n_files >= ix->replicas.size())
         return tokenize_files_group_simple(ix, n_files, file_offsets, chr, start, end, unk_id, out_file_tok, out_ids);
-    return find_host(ix, n, chr, start, end, 0, nullptr, true, n_files, file_offsets, unk_id, out_file_tok, out_ids);
+    BufPtr ids;
+    GT_TRY(find_host(ix, n, chr, start, end, 0, nullptr, true, n_files, file_offsets, unk_id, out_file_tok, &ids));
+    *out_ids = ids.release();
+    return GTGPU_OK;
 }
 
 // queries per pipeline chunk (a multiple of the tile size): 32 M on one device; a group wants at least ~4 chunks per device
@@ -627,7 +622,7 @@ int32_t tokenize_files_pipelined(gtgpu_index* gix, uint64_t n, uint64_t n_files,
 
     int32_t status = GTGPU_OK;
     cudaError_t cerr = cudaSuccess;
-    gtgpu_buf* buf = nullptr;
+    BufPtr buf;
     uint64_t* h_raw_tok = nullptr;  // pinned: every chunk's slice of raw per-file id offsets (device-local numbering)
     auto cleanup = [&]() {
         for (auto& d : devs) {
@@ -717,14 +712,7 @@ int32_t tokenize_files_pipelined(gtgpu_index* gix, uint64_t n, uint64_t n_files,
         }
         GT_CUDA(cudaSetDevice(ctx0->device));
         GT_CUDA(cudaHostAlloc((void**)&h_raw_tok, (n_files + 2) * 8, cudaHostAllocDefault));
-        buf = new gtgpu_buf();
-        buf->ctx = ctx0;
-        const int32_t s = ctx0->pinned_get(cap_total * 4, &buf->block);
-        if (s != GTGPU_OK) {
-            delete buf;
-            buf = nullptr;
-        }
-        return s;
+        return buf_new(ctx0, cap_total, 4, &buf);
     };
     status = setup();
     if (status != GTGPU_OK) {
@@ -751,51 +739,56 @@ int32_t tokenize_files_pipelined(gtgpu_index* gix, uint64_t n, uint64_t n_files,
     auto fold = [&](cudaError_t e) {
         if (cerr == cudaSuccess) cerr = e;
     };
-    for (uint64_t k = 0; k < n_chunks && status == GTGPU_OK && cerr == cudaSuccess; ++k) {
-        PipeDev& d = devs[k % D];
-        gtgpu_ctx* ctx = d.ctx;
-        cudaStream_t st = ctx->stream;
-        const uint64_t i = k / D;
-        const int b = (int)(i & 1);
-        const uint64_t q0 = k * chunk, cn = std::min(chunk, n - q0);
-        fold(cudaSetDevice(ctx->device));
-        if (i >= 2) fold(cudaStreamWaitEvent(ctx->copy_in, d.ev_free[b], 0));
-        if (!run_offsets) fold(cudaMemcpyAsync(d.in[b][0], chr + q0, cn * 4, cudaMemcpyHostToDevice, ctx->copy_in));
-        if (packed) {  // q0 is a multiple of the tile size, so the chunk starts on an anchor block
-            fold(cudaMemcpyAsync(d.in[b][1], packed + q0, cn * 4, cudaMemcpyHostToDevice, ctx->copy_in));
-            fold(cudaMemcpyAsync(d.d_anc[b], anchors + q0 / 32, (cn + 31) / 32 * 4, cudaMemcpyHostToDevice, ctx->copy_in));
-        } else {
-            fold(cudaMemcpyAsync(d.in[b][1], start + q0, cn * 4, cudaMemcpyHostToDevice, ctx->copy_in));
-            if (width16) fold(cudaMemcpyAsync(d.d_w16[b], width16 + q0, cn * 2, cudaMemcpyHostToDevice, ctx->copy_in));
-            else fold(cudaMemcpyAsync(d.in[b][2], end + q0, cn * 4, cudaMemcpyHostToDevice, ctx->copy_in));
+    try {
+        for (uint64_t k = 0; k < n_chunks && status == GTGPU_OK && cerr == cudaSuccess; ++k) {
+            PipeDev& d = devs[k % D];
+            gtgpu_ctx* ctx = d.ctx;
+            cudaStream_t st = ctx->stream;
+            const uint64_t i = k / D;
+            const int b = (int)(i & 1);
+            const uint64_t q0 = k * chunk, cn = std::min(chunk, n - q0);
+            fold(cudaSetDevice(ctx->device));
+            if (i >= 2) fold(cudaStreamWaitEvent(ctx->copy_in, d.ev_free[b], 0));
+            if (!run_offsets) fold(cudaMemcpyAsync(d.in[b][0], chr + q0, cn * 4, cudaMemcpyHostToDevice, ctx->copy_in));
+            if (packed) {  // q0 is a multiple of the tile size, so the chunk starts on an anchor block
+                fold(cudaMemcpyAsync(d.in[b][1], packed + q0, cn * 4, cudaMemcpyHostToDevice, ctx->copy_in));
+                fold(cudaMemcpyAsync(d.d_anc[b], anchors + q0 / 32, (cn + 31) / 32 * 4, cudaMemcpyHostToDevice, ctx->copy_in));
+            } else {
+                fold(cudaMemcpyAsync(d.in[b][1], start + q0, cn * 4, cudaMemcpyHostToDevice, ctx->copy_in));
+                if (width16) fold(cudaMemcpyAsync(d.d_w16[b], width16 + q0, cn * 2, cudaMemcpyHostToDevice, ctx->copy_in));
+                else fold(cudaMemcpyAsync(d.in[b][2], end + q0, cn * 4, cudaMemcpyHostToDevice, ctx->copy_in));
+            }
+            fold(cudaEventRecord(d.ev_in[b], ctx->copy_in));
+            fold(cudaStreamWaitEvent(st, d.ev_in[b], 0));
+            if (cerr != cudaSuccess) break;
+            if (packed) {
+                const uint64_t lo = std::lower_bound(wide_index, wide_index + n_wide, q0) - wide_index;
+                const uint64_t hi = std::lower_bound(wide_index, wide_index + n_wide, q0 + cn) - wide_index;
+                status = launch_expand_packed(ctx, cn, d.in[b][1], d.d_anc[b], width_bits, d.in[b][1], d.in[b][2], hi - lo, d.d_wide_idx + lo,
+                                              d.d_exc_start + lo, d.d_wide_end + lo, q0);
+            } else if (width16) {
+                const uint64_t lo = std::lower_bound(wide_index, wide_index + n_wide, q0) - wide_index;
+                const uint64_t hi = std::lower_bound(wide_index, wide_index + n_wide, q0 + cn) - wide_index;
+                status = launch_expand_widths(ctx, cn, d.in[b][1], d.d_w16[b], d.in[b][2], hi - lo, d.d_wide_idx + lo, d.d_wide_end + lo, q0);
+            }
+            if (run_offsets && status == GTGPU_OK) status = launch_expand_runs(ctx, n_runs, d.d_run_off, d.d_run_chr, q0, cn, d.in[b][0]);
+            const uint64_t L = first_f[k + 1] - first_f[k];  // file boundaries owned by this chunk
+            if (status == GTGPU_OK)
+                status = launch_fused_find(d.ix, cn, L ? L - 1 : 0, d.d_fo + first_f[k], d.in[b][0], d.in[b][1], d.in[b][2], 0, d.d_ids, d.cap,
+                                           nullptr, L ? d.d_raw_tok + first_f[k] : nullptr, d.d_ws, d.d_chain + i, d.d_chain + i + 1,
+                                           (uint32_t*)(d.d_misc + 2));
+            fold(cudaEventRecord(d.ev_free[b], st));
+            fold(cudaMemcpyAsync((void*)(ctx->h_scalars + i + 1), d.d_chain + i + 1, 8, cudaMemcpyDeviceToHost, st));
+            if (L) fold(cudaMemcpyAsync(h_raw_tok + first_f[k], d.d_raw_tok + first_f[k], L * 8, cudaMemcpyDeviceToHost, st));
+            fold(cudaEventRecord(ev_done[k], st));
+            if (k >= D) drain(k - D);  // one chunk per device stays in flight
         }
-        fold(cudaEventRecord(d.ev_in[b], ctx->copy_in));
-        fold(cudaStreamWaitEvent(st, d.ev_in[b], 0));
-        if (cerr != cudaSuccess) break;
-        if (packed) {
-            const uint64_t lo = std::lower_bound(wide_index, wide_index + n_wide, q0) - wide_index;
-            const uint64_t hi = std::lower_bound(wide_index, wide_index + n_wide, q0 + cn) - wide_index;
-            status = launch_expand_packed(ctx, cn, d.in[b][1], d.d_anc[b], width_bits, d.in[b][1], d.in[b][2], hi - lo, d.d_wide_idx + lo,
-                                          d.d_exc_start + lo, d.d_wide_end + lo, q0);
-        } else if (width16) {
-            const uint64_t lo = std::lower_bound(wide_index, wide_index + n_wide, q0) - wide_index;
-            const uint64_t hi = std::lower_bound(wide_index, wide_index + n_wide, q0 + cn) - wide_index;
-            status = launch_expand_widths(ctx, cn, d.in[b][1], d.d_w16[b], d.in[b][2], hi - lo, d.d_wide_idx + lo, d.d_wide_end + lo, q0);
-        }
-        if (run_offsets && status == GTGPU_OK) status = launch_expand_runs(ctx, n_runs, d.d_run_off, d.d_run_chr, q0, cn, d.in[b][0]);
-        const uint64_t L = first_f[k + 1] - first_f[k];  // file boundaries owned by this chunk
         if (status == GTGPU_OK)
-            status = launch_fused_find(d.ix, cn, L ? L - 1 : 0, d.d_fo + first_f[k], d.in[b][0], d.in[b][1], d.in[b][2], 0, d.d_ids, d.cap,
-                                       nullptr, L ? d.d_raw_tok + first_f[k] : nullptr, d.d_ws, d.d_chain + i, d.d_chain + i + 1,
-                                       (uint32_t*)(d.d_misc + 2));
-        fold(cudaEventRecord(d.ev_free[b], st));
-        fold(cudaMemcpyAsync((void*)(ctx->h_scalars + i + 1), d.d_chain + i + 1, 8, cudaMemcpyDeviceToHost, st));
-        if (L) fold(cudaMemcpyAsync(h_raw_tok + first_f[k], d.d_raw_tok + first_f[k], L * 8, cudaMemcpyDeviceToHost, st));
-        fold(cudaEventRecord(ev_done[k], st));
-        if (k >= D) drain(k - D);  // one chunk per device stays in flight
+            for (uint64_t j = n_chunks > D ? n_chunks - D : 0; j < n_chunks; ++j) drain(j);
+    } catch (...) {
+        cleanup();  // the copies into buf end before it goes back to the cache
+        throw;
     }
-    if (status == GTGPU_OK)
-        for (uint64_t j = n_chunks > D ? n_chunks - D : 0; j < n_chunks; ++j) drain(j);
     uint64_t total = 0, n_empty = 0;
     if (status == GTGPU_OK && cerr == cudaSuccess && !overflow) {
         for (auto& d : devs) {
@@ -817,20 +810,14 @@ int32_t tokenize_files_pipelined(gtgpu_index* gix, uint64_t n, uint64_t n_files,
         }
     }
     cleanup();
-    for (auto& d : devs) d.lock = std::unique_lock<std::mutex>();
     if (status != GTGPU_OK || cerr != cudaSuccess || overflow || n_empty > 0) {
-        {
-            std::lock_guard<std::mutex> lk(ctx0->mu);
-            ctx0->pinned_put(buf->block);
-        }
-        delete buf;
         if (status != GTGPU_OK) return status;
         if (cerr != cudaSuccess) return fail(GTGPU_ERR_CUDA, std::string("tokenize_files (pipelined): ") + cudaGetErrorString(cerr));
         *fallback = 1;
         return GTGPU_OK;
     }
     buf->len = total;
-    *out_ids = buf;
+    *out_ids = buf.release();
     return GTGPU_OK;
 }
 
@@ -861,7 +848,10 @@ int32_t gtgpu_find(gtgpu_index* ix, uint64_t n, const uint32_t* chr, const uint3
     if (!ix || !out_offsets || !out_vals || (n && (!chr || !start || !end)))
         return fail(GTGPU_ERR_INVALID, "find: null argument");
     if (is_group(ix) && n >= (1u << 16)) return find_group(ix, n, chr, start, end, min_overlap, out_offsets, out_vals);
-    return find_host(ix, n, chr, start, end, min_overlap, out_offsets, false, 0, nullptr, 0, nullptr, out_vals);
+    BufPtr vals;
+    GT_TRY(find_host(ix, n, chr, start, end, min_overlap, out_offsets, false, 0, nullptr, 0, nullptr, &vals));
+    *out_vals = vals.release();
+    return GTGPU_OK;
 } GT_CATCH
 
 int32_t gtgpu_tokenize_files(gtgpu_index* ix, uint64_t n_files, const uint64_t* file_offsets, const uint32_t* chr,

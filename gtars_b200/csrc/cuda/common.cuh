@@ -6,6 +6,7 @@
 
 #include <functional>
 #include <map>
+#include <memory>
 #include <mutex>
 #include <string>
 #include <utility>
@@ -166,6 +167,7 @@ struct gtgpu_ctx {
     int sm_count = 148;
     std::mutex mu;
     std::vector<gtgpu::DevBuffer> scratch;       // grow-only device scratch, indexed by role
+    std::mutex pinned_mu;                         // guards pinned_free; a leaf lock: nothing else is locked while it is held
     std::vector<gtgpu::PinnedBlock> pinned_free;  // cache of pinned result blocks
     uint64_t* h_scalars = nullptr;                // small pinned mailbox
     void* comm = nullptr;                         // gtgpu::Comm (NCCL), set by gtgpu_comm_init
@@ -176,7 +178,6 @@ struct gtgpu_ctx {
     std::mutex group_mu;                          // serialises group-wide calls
     bool group_comm_tried = false;                // in-process NCCL communicators (ncclCommInitAll) were set up / attempted
     int fused_bps[2][12] = {{0}, {0}};  // resident CTAs per SM of the fused find variants
-    const void* ingest_d_text = nullptr;          // set (under mu) while a *_gz entry point feeds device-resident text to the ingest
     const void* l2_window_owner = nullptr;        // the index whose window table the stream's access-policy window covers
     bool timing = false;                          // bracket dominant kernels with events
     std::vector<cudaEvent_t> ev_begin, ev_end;
@@ -184,7 +185,7 @@ struct gtgpu_ctx {
     void time_begin();
     void time_end();
     int32_t scratch_get(int role, size_t bytes, void** out);
-    int32_t pinned_get(size_t bytes, gtgpu::PinnedBlock* out);
+    int32_t pinned_get(size_t bytes, gtgpu::PinnedBlock* out);  // both take pinned_mu: callable with or without mu held
     void pinned_put(gtgpu::PinnedBlock b);
 };
 
@@ -194,6 +195,21 @@ struct gtgpu_buf {
     uint64_t len = 0;  // elements
     uint32_t elem_size = 4;
 };
+
+namespace gtgpu {
+// A result buffer the library still owns: dropping it returns the block to its ctx's cache (gtgpu_buf_free).  Hand it to the
+// caller with release() once the call can no longer fail.  A buffer with a D2H copy in flight must not be dropped before the
+// stream that carries the copy is synchronised.
+struct BufFree {
+    void operator()(gtgpu_buf* b) const { gtgpu_buf_free(b); }
+};
+using BufPtr = std::unique_ptr<gtgpu_buf, BufFree>;
+// len elements of elem_size bytes; fails with a status, never with an exception (a caller may hold a buffer with a copy in flight)
+int32_t buf_new(gtgpu_ctx* ctx, uint64_t len, uint32_t elem_size, BufPtr* out);
+// buf_new, then the D2H copy of the buffer from d_src enqueued on st, not synchronised.  A copy that cannot be enqueued fails
+// with GTGPU_ERR_CUDA and the CUDA error text alone in last_error, for the caller to put its own name in front of.
+int32_t buf_from_device(gtgpu_ctx* ctx, const void* d_src, uint64_t len, uint32_t elem_size, cudaStream_t st, BufPtr* out);
+}  // namespace gtgpu
 
 struct gtgpu_index {
     gtgpu_ctx* ctx = nullptr;
@@ -296,8 +312,7 @@ int32_t fused_find_all(gtgpu_index* ix, uint64_t nq, uint64_t n_files, const uin
 
 // fragments.cu: tokenize_fragment_file over device-resident fragments with dense barcode ids (caller holds ctx->mu)
 int32_t tokenize_fragments_core(gtgpu_index* ix, uint64_t n, const uint32_t* d_chr, const uint32_t* d_start, const uint32_t* d_end,
-                                uint32_t* d_bc, uint32_t n_barcodes, uint32_t unk_id, uint64_t* out_barcode_offsets,
-                                gtgpu_buf** out_ids);
+                                uint32_t* d_bc, uint32_t n_barcodes, uint32_t unk_id, uint64_t* out_barcode_offsets, BufPtr* out_ids);
 
 // sort.cu — hand-written scan / radix sort
 size_t exclusive_scan_temp_bytes(uint64_t n, size_t elem);
@@ -362,17 +377,18 @@ struct FragBarcodeTable {
     uint64_t n = 0, distinct = 0, cap = 0, used = 0;
     int32_t add_window(gtgpu_ctx* ctx, const char* d_text, const FragParse& fp, uint32_t n_names);
     // *out_names: the kept barcodes' bytes back to back (elem_size 1); *out_name_offsets: n_kept + 1 u64 offsets into them
-    int32_t finish(gtgpu_ctx* ctx, uint32_t* n_kept, gtgpu_buf** out_names, gtgpu_buf** out_name_offsets);
+    int32_t finish(gtgpu_ctx* ctx, uint32_t* n_kept, BufPtr* out_names, BufPtr* out_name_offsets);
 };
 // inflate.cu: H2D of gzip members + inflate; the text stays in scratch SC_GZ_OUT
 int32_t check_members(uint64_t n_members, const uint8_t* gz, const uint64_t* member_offsets, const char* who);
 int32_t gunzip_locked(gtgpu_ctx* ctx, uint64_t n_members, const uint8_t* gz, const uint64_t* member_offsets,
                       uint64_t* out_member_offsets, uint8_t** d_text, uint64_t* n_text);
-int32_t tokenize_bed_locked(gtgpu_index* ix, const char* text, uint64_t n_bytes, uint32_t n_names, const char* names,
-                            const uint32_t* name_offsets, uint32_t unk_id, gtgpu_buf** out_ids);
-int32_t tokenize_fragments_text_locked(gtgpu_index* ix, const char* text, uint64_t n_bytes, uint32_t n_names, const char* names,
-                                       const uint32_t* name_offsets, uint32_t unk_id, uint32_t* out_n_barcodes,
-                                       gtgpu_buf** out_barcode_spans, gtgpu_buf** out_barcode_offsets, gtgpu_buf** out_ids);
+// The text is host_text (copied to the device here) or dev_text (already there, e.g. inflated): exactly one is non-null.
+int32_t tokenize_bed_locked(gtgpu_index* ix, const char* host_text, const char* dev_text, uint64_t n_bytes, uint32_t n_names,
+                            const char* names, const uint32_t* name_offsets, uint32_t unk_id, gtgpu_buf** out_ids);
+int32_t tokenize_fragments_text_locked(gtgpu_index* ix, const char* host_text, const char* dev_text, uint64_t n_bytes, uint32_t n_names,
+                                       const char* names, const uint32_t* name_offsets, uint32_t unk_id, uint32_t* out_n_barcodes,
+                                       BufPtr* out_barcode_spans, BufPtr* out_barcode_offsets, BufPtr* out_ids);
 
 // groups (api.cu, comm.cu, igd.cu)
 int32_t for_each_device(size_t n_devices, const std::function<int32_t(size_t)>& fn);

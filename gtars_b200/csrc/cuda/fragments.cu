@@ -104,22 +104,12 @@ namespace gtgpu {
 
 // Device-resident core (the caller holds ctx->mu): fragments in d_chr / d_start / d_end, dense barcode ids in d_bc.
 int32_t tokenize_fragments_core(gtgpu_index* ix, uint64_t n, const uint32_t* d_chr, const uint32_t* d_start, const uint32_t* d_end,
-                                uint32_t* d_bc, uint32_t n_barcodes, uint32_t unk_id, uint64_t* out_barcode_offsets,
-                                gtgpu_buf** out_ids) {
+                                uint32_t* d_bc, uint32_t n_barcodes, uint32_t unk_id, uint64_t* out_barcode_offsets, BufPtr* out_ids) {
     gtgpu_ctx* ctx = ix->ctx;
     cudaStream_t st = ctx->stream;
     if (n == 0) {
         for (uint32_t b = 0; b <= n_barcodes; ++b) out_barcode_offsets[b] = 0;
-        gtgpu_buf* buf = new gtgpu_buf();
-        buf->ctx = ctx;
-        buf->len = 0;
-        const int32_t s = ctx->pinned_get(0, &buf->block);
-        if (s != GTGPU_OK) {
-            delete buf;
-            return s;
-        }
-        *out_ids = buf;
-        return GTGPU_OK;
+        return buf_new(ctx, 0, 4, out_ids);
     }
     uint32_t *d_out = nullptr, *d_alt = nullptr, *d_tag_a = nullptr, *d_tag_b = nullptr;
     uint64_t *d_off, *d_bco, *d_misc;
@@ -153,23 +143,13 @@ int32_t tokenize_fragments_core(gtgpu_index* ix, uint64_t n, const uint32_t* d_c
                               d_tmp, d_misc, d_bco, nullptr, 2, &tag_if));
     GT_CUDA(cudaMemcpyAsync(out_barcode_offsets, d_bco, ((uint64_t)n_barcodes + 1) * 8, cudaMemcpyDeviceToHost, st));
 
-    gtgpu_buf* buf = new gtgpu_buf();
-    buf->ctx = ctx;
-    buf->len = total;
-    int32_t s = ctx->pinned_get(total * 4, &buf->block);
-    if (s != GTGPU_OK) {
-        delete buf;
-        return s;
-    }
-    cudaError_t e = cudaSuccess;
-    if (total) e = cudaMemcpyAsync(buf->block.ptr, d_out, total * 4, cudaMemcpyDeviceToHost, st);
-    if (e == cudaSuccess) e = cudaStreamSynchronize(st);
-    if (e != cudaSuccess) {
-        ctx->pinned_put(buf->block);
-        delete buf;
-        return fail(GTGPU_ERR_CUDA, std::string("tokenize_fragments: D2H: ") + cudaGetErrorString(e));
-    }
-    *out_ids = buf;
+    BufPtr buf;
+    const int32_t s = buf_from_device(ctx, d_out, total, 4, st, &buf);
+    if (s == GTGPU_ERR_CUDA) return fail(s, std::string("tokenize_fragments: D2H: ") + gtgpu_last_error());
+    GT_TRY(s);
+    const cudaError_t e = cudaStreamSynchronize(st);
+    if (e != cudaSuccess) return fail(GTGPU_ERR_CUDA, std::string("tokenize_fragments: D2H: ") + cudaGetErrorString(e));
+    *out_ids = std::move(buf);
     return GTGPU_OK;
 }
 
@@ -177,7 +157,7 @@ int32_t tokenize_fragments_core(gtgpu_index* ix, uint64_t n, const uint32_t* d_c
 
 static int32_t tokenize_fragments_one(gtgpu_index* ix, uint64_t n, const uint32_t* chr, const uint32_t* start, const uint32_t* end,
                                       const uint32_t* barcode_id, uint32_t n_barcodes, uint32_t unk_id,
-                                      uint64_t* out_barcode_offsets, gtgpu_buf** out_ids) {
+                                      uint64_t* out_barcode_offsets, BufPtr* out_ids) {
     gtgpu_ctx* ctx = ix->ctx;
     std::lock_guard<std::mutex> lk(ctx->mu);
     GT_CUDA(cudaSetDevice(ctx->device));
@@ -204,7 +184,7 @@ static int32_t tokenize_fragments_group(gtgpu_index* ix, uint64_t n, const uint3
                                         uint64_t* out_barcode_offsets, gtgpu_buf** out_ids) {
     std::lock_guard<std::mutex> glk(ix->ctx->group_mu);
     const size_t D = ix->replicas.size();
-    std::vector<gtgpu_buf*> parts(D, nullptr);
+    std::vector<BufPtr> parts(D);
     std::vector<std::vector<uint64_t>> offs(D, std::vector<uint64_t>((size_t)n_barcodes + 1, 0));
     int32_t s = for_each_device(D, [&](size_t r) -> int32_t {
         uint64_t lo, hi;
@@ -212,7 +192,7 @@ static int32_t tokenize_fragments_group(gtgpu_index* ix, uint64_t n, const uint3
         return tokenize_fragments_one(ix->replicas[r], hi - lo, chr + lo, start + lo, end + lo, barcode_id + lo, n_barcodes, unk_id,
                                       offs[r].data(), &parts[r]);
     });
-    gtgpu_buf* buf = nullptr;
+    BufPtr buf;
     if (s == GTGPU_OK) {
         out_barcode_offsets[0] = 0;
         for (uint32_t b = 0; b < n_barcodes; ++b) {
@@ -220,18 +200,8 @@ static int32_t tokenize_fragments_group(gtgpu_index* ix, uint64_t n, const uint3
             for (size_t r = 0; r < D; ++r) len += offs[r][b + 1] - offs[r][b];
             out_barcode_offsets[b + 1] = out_barcode_offsets[b] + len;
         }
-        buf = new gtgpu_buf();
-        buf->ctx = ix->ctx;
-        buf->len = out_barcode_offsets[n_barcodes];
-        {
-            std::lock_guard<std::mutex> lk(ix->ctx->mu);
-            cudaSetDevice(ix->ctx->device);
-            s = ix->ctx->pinned_get(buf->len * 4, &buf->block);
-        }
-        if (s != GTGPU_OK) {
-            delete buf;
-            buf = nullptr;
-        }
+        cudaSetDevice(ix->ctx->device);
+        s = buf_new(ix->ctx, out_barcode_offsets[n_barcodes], 4, &buf);
     }
     if (s == GTGPU_OK) {
         uint32_t* dst = (uint32_t*)buf->block.ptr;
@@ -248,10 +218,8 @@ static int32_t tokenize_fragments_group(gtgpu_index* ix, uint64_t n, const uint3
             }
             return GTGPU_OK;
         });
-        *out_ids = buf;
+        *out_ids = buf.release();
     }
-    for (auto* p : parts)
-        if (p) gtgpu_buf_free(p);
     return s;
 }
 
@@ -265,7 +233,10 @@ extern "C" int32_t gtgpu_tokenize_fragments(gtgpu_index* ix, uint64_t n, const u
         if (barcode_id[i] >= n_barcodes) return fail(GTGPU_ERR_INVALID, "tokenize_fragments: barcode id out of range");
     if (ix->replicas.size() > 1 && n >= (1u << 20))
         return tokenize_fragments_group(ix, n, chr, start, end, barcode_id, n_barcodes, unk_id, out_barcode_offsets, out_ids);
-    return tokenize_fragments_one(ix, n, chr, start, end, barcode_id, n_barcodes, unk_id, out_barcode_offsets, out_ids);
+    BufPtr ids;
+    GT_TRY(tokenize_fragments_one(ix, n, chr, start, end, barcode_id, n_barcodes, unk_id, out_barcode_offsets, &ids));
+    *out_ids = ids.release();
+    return GTGPU_OK;
 } GT_CATCH
 
 // Device-resident form of gtgpu_tokenize_fragments: nothing crosses PCIe and nothing synchronises — find, tagging, the

@@ -619,12 +619,6 @@ int32_t check_members(uint64_t n_members, const uint8_t* gz, const uint64_t* mem
     return GTGPU_OK;
 }
 
-struct IngestTextScope {  // ctx->ingest_d_text for the duration of one locked call
-    gtgpu_ctx* ctx;
-    IngestTextScope(gtgpu_ctx* c, const void* p) : ctx(c) { ctx->ingest_d_text = p; }
-    ~IngestTextScope() { ctx->ingest_d_text = nullptr; }
-};
-
 }  // namespace gtgpu
 
 extern "C" int32_t gtgpu_gunzip(gtgpu_ctx* ctx, uint64_t n_members, const uint8_t* gz, const uint64_t* member_offsets,
@@ -636,23 +630,13 @@ extern "C" int32_t gtgpu_gunzip(gtgpu_ctx* ctx, uint64_t n_members, const uint8_
     uint8_t* d_text = nullptr;
     uint64_t n_text = 0;
     GT_TRY(gunzip_locked(ctx, n_members, gz, member_offsets, out_member_offsets, &d_text, &n_text));
-    gtgpu_buf* buf = new gtgpu_buf();
-    buf->ctx = ctx;
-    buf->len = n_text;
-    buf->elem_size = 1;
-    const int32_t s = ctx->pinned_get(n_text, &buf->block);
-    if (s != GTGPU_OK) {
-        delete buf;
-        return s;
-    }
-    cudaError_t e = n_text ? cudaMemcpyAsync(buf->block.ptr, d_text, n_text, cudaMemcpyDeviceToHost, ctx->stream) : cudaSuccess;
-    if (e == cudaSuccess) e = cudaStreamSynchronize(ctx->stream);
-    if (e != cudaSuccess) {
-        ctx->pinned_put(buf->block);
-        delete buf;
-        return fail(GTGPU_ERR_CUDA, std::string("gunzip: D2H: ") + cudaGetErrorString(e));
-    }
-    *out_text = buf;
+    BufPtr buf;
+    const int32_t s = buf_from_device(ctx, d_text, n_text, 1, ctx->stream, &buf);
+    if (s == GTGPU_ERR_CUDA) return fail(s, std::string("gunzip: D2H: ") + gtgpu_last_error());
+    GT_TRY(s);
+    const cudaError_t e = cudaStreamSynchronize(ctx->stream);
+    if (e != cudaSuccess) return fail(GTGPU_ERR_CUDA, std::string("gunzip: D2H: ") + cudaGetErrorString(e));
+    *out_text = buf.release();
     return GTGPU_OK;
 } GT_CATCH
 
@@ -668,8 +652,7 @@ extern "C" int32_t gtgpu_tokenize_bed_gz(gtgpu_index* ix, uint64_t n_members, co
     uint8_t* d_text = nullptr;
     uint64_t n_text = 0;
     GT_TRY(gunzip_locked(ctx, n_members, gz, member_offsets, nullptr, &d_text, &n_text));
-    IngestTextScope scope(ctx, d_text);
-    return tokenize_bed_locked(ix, nullptr, n_text, n_names, names, name_offsets, unk_id, out_ids);
+    return tokenize_bed_locked(ix, nullptr, (const char*)d_text, n_text, n_names, names, name_offsets, unk_id, out_ids);
 } GT_CATCH
 
 // gtgpu_tokenize_fragments_text on gzip members (a bgzip'ed fragment file: thousands of members).  *out_text returns the
@@ -688,25 +671,25 @@ extern "C" int32_t gtgpu_tokenize_fragments_gz(gtgpu_index* ix, uint64_t n_membe
     uint8_t* d_text = nullptr;
     uint64_t n_text = 0;
     GT_TRY(gunzip_locked(ctx, n_members, gz, member_offsets, nullptr, &d_text, &n_text));
-    gtgpu_buf* text = new gtgpu_buf();
-    text->ctx = ctx;
-    text->len = n_text;
-    text->elem_size = 1;
-    int32_t s = ctx->pinned_get(n_text, &text->block);
-    if (s == GTGPU_OK && n_text && cudaMemcpyAsync(text->block.ptr, d_text, n_text, cudaMemcpyDeviceToHost, ctx->copy_out) != cudaSuccess)
-        s = fail(GTGPU_ERR_CUDA, "tokenize_fragments_gz: D2H of the text failed");
-    if (s == GTGPU_OK) {
-        IngestTextScope scope(ctx, d_text);
-        s = tokenize_fragments_text_locked(ix, nullptr, n_text, n_names, names, name_offsets, unk_id, out_n_barcodes, out_barcode_spans,
-                                           out_barcode_offsets, out_ids);
+    BufPtr text, spans, offs, ids;  // the text's copy on copy_out overlaps the parse
+    int32_t s = buf_from_device(ctx, d_text, n_text, 1, ctx->copy_out, &text);
+    if (s == GTGPU_ERR_CUDA) return fail(s, "tokenize_fragments_gz: D2H of the text failed");
+    GT_TRY(s);
+    try {
+        s = tokenize_fragments_text_locked(ix, nullptr, (const char*)d_text, n_text, n_names, names, name_offsets, unk_id, out_n_barcodes,
+                                           &spans, &offs, &ids);
+    } catch (...) {
+        cudaStreamSynchronize(ctx->copy_out);  // the text's copy ends before its block goes back to the cache
+        throw;
     }
     if (s == GTGPU_OK && cudaStreamSynchronize(ctx->copy_out) != cudaSuccess) s = fail(GTGPU_ERR_CUDA, "tokenize_fragments_gz: D2H of the text failed");
     if (s != GTGPU_OK) {
         cudaStreamSynchronize(ctx->copy_out);
-        if (text->block.ptr) ctx->pinned_put(text->block);
-        delete text;
         return s;
     }
-    *out_text = text;
+    *out_barcode_spans = spans.release();
+    *out_barcode_offsets = offs.release();
+    *out_ids = ids.release();
+    *out_text = text.release();
     return GTGPU_OK;
 } GT_CATCH

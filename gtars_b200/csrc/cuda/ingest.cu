@@ -553,10 +553,10 @@ int32_t parse_fragments_locked(gtgpu_ctx* ctx, const char* d_text, uint64_t n_by
 }
 
 // Parses and sorts on the device.  On success *d_chr / *d_start / *d_end point at n_out regions in device scratch
-// (valid until the next call on this ctx).  The caller holds ctx->mu.
-static int32_t parse_bed_locked(gtgpu_ctx* ctx, const char* text, uint64_t n_bytes, uint32_t n_names, const char* names,
-                                const uint32_t* name_offsets, uint64_t* n_out, uint32_t** d_chr, uint32_t** d_start,
-                                uint32_t** d_end) {
+// (valid until the next call on this ctx).  Exactly one of host_text / dev_text is given.  The caller holds ctx->mu.
+static int32_t parse_bed_locked(gtgpu_ctx* ctx, const char* host_text, const char* dev_text, uint64_t n_bytes, uint32_t n_names,
+                                const char* names, const uint32_t* name_offsets, uint64_t* n_out, uint32_t** d_chr,
+                                uint32_t** d_start, uint32_t** d_end) {
     if (n_bytes >= 0xFFFFFFF0ull) return fail(GTGPU_ERR_UNSUPPORTED, "parse_bed: at most 4 GiB of text per call (split at a line boundary)");
     if (n_names >= 0x7FFFFFFFu) return fail(GTGPU_ERR_INVALID, "parse_bed: too many chromosome names");
     cudaStream_t st = ctx->stream;
@@ -581,19 +581,17 @@ static int32_t parse_bed_locked(gtgpu_ctx* ctx, const char* text, uint64_t n_byt
     for (uint32_t r = 0; r < n_names; ++r) rank[by_name[r]] = r;  // equal strings cannot occur in a name table
     const uint32_t blob_bytes = n_names ? name_offsets[n_names] : 0;
 
-    char* d_text;
+    const char* d_text = dev_text;
     uint32_t *d_counts, *d_crank, *d_nl;
     void* d_tmp;
     char* d_names;
     const uint64_t n_chunks = (n_bytes + INGEST_CHUNK - 1) / INGEST_CHUNK;
-    // the text is either the caller's host buffer or already on the device (gtgpu_*_gz: inflated there, ctx->ingest_d_text)
-    if (ctx->ingest_d_text) d_text = (char*)ctx->ingest_d_text;
-    else GT_TRY(ctx->scratch_get(SC_OUT_IDS2, n_bytes + 64, (void**)&d_text));
+    if (!dev_text) GT_TRY(ctx->scratch_get(SC_OUT_IDS2, n_bytes + 64, (void**)&d_text));
     GT_TRY(ctx->scratch_get(SC_COUNTS, n_chunks * 4 + 4, (void**)&d_counts));
     GT_TRY(ctx->scratch_get(SC_IN3_CHR, n_chunks * 4 + 4, (void**)&d_crank));
     const size_t names_bytes = ((size_t)blob_bytes + 15) / 16 * 16 + ((size_t)n_names + 1) * 4 + (size_t)n_names * 8 + (size_t)n_names * 4 * 2 + 64;
     GT_TRY(ctx->scratch_get(SC_SET_ID, names_bytes, (void**)&d_names));
-    if (!ctx->ingest_d_text) GT_CUDA(cudaMemcpyAsync(d_text, text, n_bytes, cudaMemcpyHostToDevice, st));
+    if (!dev_text) GT_CUDA(cudaMemcpyAsync((char*)d_text, host_text, n_bytes, cudaMemcpyHostToDevice, st));
     // layout of the name scratch: hashes (8-byte aligned first), offsets, hash ids, ranks, blob
     unsigned long long* d_hash = reinterpret_cast<unsigned long long*>(d_names);
     uint32_t* d_noff = reinterpret_cast<uint32_t*>(d_hash + n_names);
@@ -778,7 +776,7 @@ int32_t FragBarcodeTable::add_window(gtgpu_ctx* ctx, const char* d_text, const F
     return GTGPU_OK;
 }
 
-int32_t FragBarcodeTable::finish(gtgpu_ctx* ctx, uint32_t* n_kept, gtgpu_buf** out_names, gtgpu_buf** out_name_offsets) {
+int32_t FragBarcodeTable::finish(gtgpu_ctx* ctx, uint32_t* n_kept, BufPtr* out_names, BufPtr* out_name_offsets) {
     cudaStream_t st = ctx->stream;
     uint64_t kept = 0, blob_bytes = 0;
     char* d_blob = nullptr;
@@ -816,51 +814,22 @@ int32_t FragBarcodeTable::finish(gtgpu_ctx* ctx, uint32_t* n_kept, gtgpu_buf** o
         ctx->launches++;
         GT_CUDA(cudaGetLastError());
     }
-    gtgpu_buf* bufs[2] = {new gtgpu_buf(), new gtgpu_buf()};
-    const uint64_t lens[2] = {blob_bytes, kept + 1};
-    int32_t s = GTGPU_OK;
-    for (int k = 0; k < 2; ++k) {
-        bufs[k]->ctx = ctx;
-        bufs[k]->len = lens[k];
-        bufs[k]->elem_size = k == 0 ? 1 : 8;
-        if (s == GTGPU_OK) s = ctx->pinned_get(lens[k] * bufs[k]->elem_size, &bufs[k]->block);
-    }
-    if (s == GTGPU_OK && blob_bytes && cudaMemcpyAsync(bufs[0]->block.ptr, d_blob, blob_bytes, cudaMemcpyDeviceToHost, st) != cudaSuccess)
-        s = fail(GTGPU_ERR_CUDA, "score_barcodes_text: D2H of the barcode names failed");
-    if (s == GTGPU_OK && kept && cudaMemcpyAsync(bufs[1]->block.ptr, d_noff, kept * 8, cudaMemcpyDeviceToHost, st) != cudaSuccess)
+    BufPtr names, offsets;
+    int32_t s = buf_from_device(ctx, d_blob, blob_bytes, 1, st, &names);
+    if (s == GTGPU_ERR_CUDA) return fail(s, "score_barcodes_text: D2H of the barcode names failed");
+    GT_TRY(s);
+    s = buf_new(ctx, kept + 1, 8, &offsets);  // the last offset is written on the host
+    if (s == GTGPU_OK && kept && cudaMemcpyAsync(offsets->block.ptr, d_noff, kept * 8, cudaMemcpyDeviceToHost, st) != cudaSuccess)
         s = fail(GTGPU_ERR_CUDA, "score_barcodes_text: D2H of the barcode name offsets failed");
     if (s == GTGPU_OK && cudaStreamSynchronize(st) != cudaSuccess) s = fail(GTGPU_ERR_CUDA, "score_barcodes_text: D2H failed");
     if (s != GTGPU_OK) {
-        for (auto* b : bufs) {
-            if (b->block.ptr) ctx->pinned_put(b->block);
-            delete b;
-        }
+        cudaStreamSynchronize(st);  // the names' copy may still run
         return s;
     }
-    reinterpret_cast<uint64_t*>(bufs[1]->block.ptr)[kept] = blob_bytes;
+    reinterpret_cast<uint64_t*>(offsets->block.ptr)[kept] = blob_bytes;
     *n_kept = (uint32_t)kept;
-    *out_names = bufs[0];
-    *out_name_offsets = bufs[1];
-    return GTGPU_OK;
-}
-
-static int32_t to_host_buf(gtgpu_ctx* ctx, const uint32_t* d_src, uint64_t n, gtgpu_buf** out) {
-    gtgpu_buf* buf = new gtgpu_buf();
-    buf->ctx = ctx;
-    buf->len = n;
-    int32_t s = ctx->pinned_get(n * 4, &buf->block);
-    if (s != GTGPU_OK) {
-        delete buf;
-        return s;
-    }
-    cudaError_t e = n ? cudaMemcpyAsync(buf->block.ptr, d_src, n * 4, cudaMemcpyDeviceToHost, ctx->stream) : cudaSuccess;
-    if (e == cudaSuccess) e = cudaStreamSynchronize(ctx->stream);
-    if (e != cudaSuccess) {
-        ctx->pinned_put(buf->block);
-        delete buf;
-        return fail(GTGPU_ERR_CUDA, std::string("ingest: D2H: ") + cudaGetErrorString(e));
-    }
-    *out = buf;
+    *out_names = std::move(names);
+    *out_name_offsets = std::move(offsets);
     return GTGPU_OK;
 }
 
@@ -877,20 +846,20 @@ extern "C" int32_t gtgpu_parse_bed(gtgpu_ctx* ctx, const char* text, uint64_t n_
     GT_CUDA(cudaSetDevice(ctx->device));
     uint32_t *d_chr, *d_start, *d_end;
     uint64_t n = 0;
-    GT_TRY(parse_bed_locked(ctx, text, n_bytes, n_names, names, name_offsets, &n, &d_chr, &d_start, &d_end));
-    gtgpu_buf* bufs[3] = {nullptr, nullptr, nullptr};
+    GT_TRY(parse_bed_locked(ctx, text, nullptr, n_bytes, n_names, names, name_offsets, &n, &d_chr, &d_start, &d_end));
+    BufPtr bufs[3];
     const uint32_t* src[3] = {d_chr, d_start, d_end};
     for (int k = 0; k < 3; ++k) {
-        int32_t s = to_host_buf(ctx, src[k], n, &bufs[k]);
-        if (s != GTGPU_OK) {
-            for (int j = 0; j < k; ++j) { ctx->pinned_put(bufs[j]->block); delete bufs[j]; }
-            return s;
-        }
+        const int32_t s = buf_from_device(ctx, src[k], n, 4, ctx->stream, &bufs[k]);
+        if (s == GTGPU_ERR_CUDA) return fail(s, std::string("ingest: D2H: ") + gtgpu_last_error());
+        GT_TRY(s);
+        const cudaError_t e = cudaStreamSynchronize(ctx->stream);
+        if (e != cudaSuccess) return fail(GTGPU_ERR_CUDA, std::string("ingest: D2H: ") + cudaGetErrorString(e));
     }
     *out_n = n;
-    *out_chr = bufs[0];
-    *out_start = bufs[1];
-    *out_end = bufs[2];
+    *out_chr = bufs[0].release();
+    *out_start = bufs[1].release();
+    *out_end = bufs[2].release();
     return GTGPU_OK;
 } GT_CATCH
 
@@ -901,31 +870,31 @@ extern "C" int32_t gtgpu_tokenize_bed(gtgpu_index* ix, const char* text, uint64_
     gtgpu_ctx* ctx = ix->ctx;
     std::lock_guard<std::mutex> lk(ctx->mu);
     GT_CUDA(cudaSetDevice(ctx->device));
-    return tokenize_bed_locked(ix, text, n_bytes, n_names, names, name_offsets, unk_id, out_ids);
+    return tokenize_bed_locked(ix, text, nullptr, n_bytes, n_names, names, name_offsets, unk_id, out_ids);
 } GT_CATCH
 
-// the caller holds ctx->mu; `text` is ignored when ctx->ingest_d_text points at the text on the device
-int32_t gtgpu::tokenize_bed_locked(gtgpu_index* ix, const char* text, uint64_t n_bytes, uint32_t n_names, const char* names,
-                                   const uint32_t* name_offsets, uint32_t unk_id, gtgpu_buf** out_ids) {
+// the caller holds ctx->mu
+int32_t gtgpu::tokenize_bed_locked(gtgpu_index* ix, const char* host_text, const char* dev_text, uint64_t n_bytes, uint32_t n_names,
+                                   const char* names, const uint32_t* name_offsets, uint32_t unk_id, gtgpu_buf** out_ids) {
     gtgpu_ctx* ctx = ix->ctx;
     uint32_t *d_chr, *d_start, *d_end, *d_ids = nullptr;
     uint64_t n = 0, total = 0;
-    GT_TRY(parse_bed_locked(ctx, text, n_bytes, n_names, names, name_offsets, &n, &d_chr, &d_start, &d_end));
+    GT_TRY(parse_bed_locked(ctx, host_text, dev_text, n_bytes, n_names, names, name_offsets, &n, &d_chr, &d_start, &d_end));
     GT_TRY(fused_find_all(ix, n, 0, nullptr, d_chr, d_start, d_end, nullptr, nullptr, &d_ids, &total));
+    BufPtr buf;
     if (total == 0) {  // Tokenizer::tokenize: a call without a single token yields [unk] (tokenizer.rs:156-160)
-        gtgpu_buf* buf = new gtgpu_buf();
-        buf->ctx = ctx;
-        buf->len = 1;
-        int32_t s = ctx->pinned_get(4, &buf->block);
-        if (s != GTGPU_OK) {
-            delete buf;
-            return s;
-        }
+        GT_TRY(buf_new(ctx, 1, 4, &buf));
         *reinterpret_cast<uint32_t*>(buf->block.ptr) = unk_id;
-        *out_ids = buf;
+        *out_ids = buf.release();
         return GTGPU_OK;
     }
-    return to_host_buf(ctx, d_ids, total, out_ids);
+    const int32_t s = buf_from_device(ctx, d_ids, total, 4, ctx->stream, &buf);
+    if (s == GTGPU_ERR_CUDA) return fail(s, std::string("ingest: D2H: ") + gtgpu_last_error());
+    GT_TRY(s);
+    const cudaError_t e = cudaStreamSynchronize(ctx->stream);
+    if (e != cudaSuccess) return fail(GTGPU_ERR_CUDA, std::string("ingest: D2H: ") + cudaGetErrorString(e));
+    *out_ids = buf.release();
+    return GTGPU_OK;
 }
 
 // tokenize_fragment_file (fragments.rs:61-82) from the file's text: parse on the device, barcodes -> dense ids in
@@ -940,14 +909,20 @@ extern "C" int32_t gtgpu_tokenize_fragments_text(gtgpu_index* ix, const char* te
     gtgpu_ctx* ctx = ix->ctx;
     std::lock_guard<std::mutex> lk(ctx->mu);
     GT_CUDA(cudaSetDevice(ctx->device));
-    return tokenize_fragments_text_locked(ix, text, n_bytes, n_names, names, name_offsets, unk_id, out_n_barcodes, out_barcode_spans,
-                                          out_barcode_offsets, out_ids);
+    BufPtr spans, offs, ids;
+    GT_TRY(tokenize_fragments_text_locked(ix, text, nullptr, n_bytes, n_names, names, name_offsets, unk_id, out_n_barcodes, &spans,
+                                          &offs, &ids));
+    *out_barcode_spans = spans.release();
+    *out_barcode_offsets = offs.release();
+    *out_ids = ids.release();
+    return GTGPU_OK;
 } GT_CATCH
 
-// the caller holds ctx->mu; `text` is ignored when ctx->ingest_d_text points at the text on the device
-int32_t gtgpu::tokenize_fragments_text_locked(gtgpu_index* ix, const char* text, uint64_t n_bytes, uint32_t n_names, const char* names,
-                                              const uint32_t* name_offsets, uint32_t unk_id, uint32_t* out_n_barcodes,
-                                              gtgpu_buf** out_barcode_spans, gtgpu_buf** out_barcode_offsets, gtgpu_buf** out_ids) {
+// the caller holds ctx->mu
+int32_t gtgpu::tokenize_fragments_text_locked(gtgpu_index* ix, const char* host_text, const char* dev_text, uint64_t n_bytes,
+                                              uint32_t n_names, const char* names, const uint32_t* name_offsets, uint32_t unk_id,
+                                              uint32_t* out_n_barcodes, BufPtr* out_barcode_spans, BufPtr* out_barcode_offsets,
+                                              BufPtr* out_ids) {
     if (n_bytes >= 0xFFFFFFF0ull) return fail(GTGPU_ERR_UNSUPPORTED, "tokenize_fragments_text: at most 4 GiB of text per call");
     gtgpu_ctx* ctx = ix->ctx;
     cudaStream_t st = ctx->stream;
@@ -957,10 +932,9 @@ int32_t gtgpu::tokenize_fragments_text_locked(gtgpu_index* ix, const char* text,
     if (n_bytes) {
         NameTable nt;
         GT_TRY(upload_name_table(ctx, n_names, names, name_offsets, &nt));
-        char* d_text;
-        if (ctx->ingest_d_text) d_text = (char*)ctx->ingest_d_text;
-        else GT_TRY(ctx->scratch_get(SC_OUT_IDS2, n_bytes + 64, (void**)&d_text));
-        if (!ctx->ingest_d_text) GT_CUDA(cudaMemcpyAsync(d_text, text, n_bytes, cudaMemcpyHostToDevice, st));
+        const char* d_text = dev_text;
+        if (!dev_text) GT_TRY(ctx->scratch_get(SC_OUT_IDS2, n_bytes + 64, (void**)&d_text));
+        if (!dev_text) GT_CUDA(cudaMemcpyAsync((char*)d_text, host_text, n_bytes, cudaMemcpyHostToDevice, st));
         FragParse fp;
         GT_TRY(parse_fragments_locked(ctx, d_text, n_bytes, nt, FRAG_TOKENIZE, &fp));
         if (fp.bad_line != 0xFFFFFFFFu)
@@ -999,31 +973,21 @@ int32_t gtgpu::tokenize_fragments_text_locked(gtgpu_index* ix, const char* text,
     }
     // ---- results -----------------------------------------------------------------------------------------------------------------
     *out_n_barcodes = n_barcodes;
-    gtgpu_buf* spans = nullptr;
-    GT_TRY(to_host_buf(ctx, d_spans, (uint64_t)n_barcodes * 2, &spans));
-    gtgpu_buf* offs = new gtgpu_buf();
-    offs->ctx = ctx;
-    offs->len = (uint64_t)n_barcodes + 1;
-    offs->elem_size = 8;
-    int32_t status = ctx->pinned_get(offs->len * 8, &offs->block);
-    gtgpu_buf* ids = nullptr;
-    if (status == GTGPU_OK) {
-        if (n) {
-            status = tokenize_fragments_core(ix, n, o_chr, o_start, o_end, d_bcid, n_barcodes, unk_id, (uint64_t*)offs->block.ptr, &ids);
-        } else {
-            *(uint64_t*)offs->block.ptr = 0;
-            status = to_host_buf(ctx, nullptr, 0, &ids);
-        }
+    BufPtr spans, offs, ids;
+    const int32_t s = buf_from_device(ctx, d_spans, (uint64_t)n_barcodes * 2, 4, st, &spans);
+    if (s == GTGPU_ERR_CUDA) return fail(s, std::string("ingest: D2H: ") + gtgpu_last_error());
+    GT_TRY(s);
+    const cudaError_t e = cudaStreamSynchronize(st);
+    if (e != cudaSuccess) return fail(GTGPU_ERR_CUDA, std::string("ingest: D2H: ") + cudaGetErrorString(e));
+    GT_TRY(buf_new(ctx, (uint64_t)n_barcodes + 1, 8, &offs));
+    if (n) {
+        GT_TRY(tokenize_fragments_core(ix, n, o_chr, o_start, o_end, d_bcid, n_barcodes, unk_id, (uint64_t*)offs->block.ptr, &ids));
+    } else {
+        *(uint64_t*)offs->block.ptr = 0;
+        GT_TRY(buf_new(ctx, 0, 4, &ids));
     }
-    if (status != GTGPU_OK) {
-        ctx->pinned_put(spans->block);
-        delete spans;
-        if (offs->block.ptr) ctx->pinned_put(offs->block);
-        delete offs;
-        return status;
-    }
-    *out_barcode_spans = spans;
-    *out_barcode_offsets = offs;
-    *out_ids = ids;
+    *out_barcode_spans = std::move(spans);
+    *out_barcode_offsets = std::move(offs);
+    *out_ids = std::move(ids);
     return GTGPU_OK;
 }

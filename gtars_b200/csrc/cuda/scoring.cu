@@ -324,30 +324,17 @@ static int32_t score_barcodes_dev_locked(gtgpu_index* ix, uint64_t n, const uint
     if (nnz == 0)
         for (uint32_t b = 0; b <= n_barcodes; ++b) out_barcode_offsets[b] = 0;
 
-    gtgpu_buf* bufs[2] = {nullptr, nullptr};
-    const uint32_t* srcs[2] = {d_peak_out, d_count_out};
-    for (int k = 0; k < 2; ++k) {
-        gtgpu_buf* buf = new gtgpu_buf();
-        buf->ctx = ctx;
-        buf->len = nnz;
-        int32_t s = ctx->pinned_get(nnz * 4, &buf->block);
-        cudaError_t e = cudaSuccess;
-        if (s == GTGPU_OK && nnz) e = cudaMemcpyAsync(buf->block.ptr, srcs[k], nnz * 4, cudaMemcpyDeviceToHost, st);
-        if (s != GTGPU_OK || e != cudaSuccess) {
-            if (s == GTGPU_OK) ctx->pinned_put(buf->block);
-            delete buf;
-            if (bufs[0]) { ctx->pinned_put(bufs[0]->block); delete bufs[0]; }
-            return s != GTGPU_OK ? s : fail(GTGPU_ERR_CUDA, std::string("score_barcodes: D2H: ") + cudaGetErrorString(e));
-        }
-        bufs[k] = buf;
+    BufPtr peaks, counts;
+    int32_t s = buf_from_device(ctx, d_peak_out, nnz, 4, st, &peaks);
+    if (s == GTGPU_OK) s = buf_from_device(ctx, d_count_out, nnz, 4, st, &counts);
+    if (s != GTGPU_OK) {
+        cudaStreamSynchronize(st);  // the peaks' copy may still run
+        return s == GTGPU_ERR_CUDA ? fail(s, std::string("score_barcodes: D2H: ") + gtgpu_last_error()) : s;
     }
-    cudaError_t e = cudaStreamSynchronize(st);
-    if (e != cudaSuccess) {
-        for (auto* b : bufs) { ctx->pinned_put(b->block); delete b; }
-        return fail(GTGPU_ERR_CUDA, std::string("score_barcodes: ") + cudaGetErrorString(e));
-    }
-    *out_peaks = bufs[0];
-    *out_counts = bufs[1];
+    const cudaError_t e = cudaStreamSynchronize(st);
+    if (e != cudaSuccess) return fail(GTGPU_ERR_CUDA, std::string("score_barcodes: ") + cudaGetErrorString(e));
+    *out_peaks = peaks.release();
+    *out_counts = counts.release();
     return GTGPU_OK;
 }
 
@@ -565,27 +552,15 @@ static int32_t score_barcodes_text_locked(gtgpu_index* ix, const char* host_text
         }));
     }
     uint32_t n_kept = 0;
-    gtgpu_buf *nm = nullptr, *no = nullptr;
+    BufPtr nm, no, offs;
     GT_TRY(tab.finish(ctx, &n_kept, &nm, &no));
-    gtgpu_buf* offs = new gtgpu_buf();
-    offs->ctx = ctx;
-    offs->len = (uint64_t)n_kept + 1;
-    offs->elem_size = 8;
-    int32_t s = ctx->pinned_get(offs->len * 8, &offs->block);
-    if (s == GTGPU_OK)
-        s = score_barcodes_dev_locked(ix, tab.n, tab.chr.u32(), tab.start.u32(), tab.end.u32(), tab.bc.u32(), n_kept,
-                                      (uint64_t*)offs->block.ptr, out_peaks, out_counts);
-    if (s != GTGPU_OK) {
-        for (gtgpu_buf* b : {nm, no, offs}) {
-            if (b->block.ptr) ctx->pinned_put(b->block);
-            delete b;
-        }
-        return s;
-    }
+    GT_TRY(buf_new(ctx, (uint64_t)n_kept + 1, 8, &offs));
+    GT_TRY(score_barcodes_dev_locked(ix, tab.n, tab.chr.u32(), tab.start.u32(), tab.end.u32(), tab.bc.u32(), n_kept,
+                                     (uint64_t*)offs->block.ptr, out_peaks, out_counts));
     *out_n_barcodes = n_kept;
-    *out_names = nm;
-    *out_name_offsets = no;
-    *out_barcode_offsets = offs;
+    *out_names = nm.release();
+    *out_name_offsets = no.release();
+    *out_barcode_offsets = offs.release();
     return GTGPU_OK;
 }
 
