@@ -361,8 +361,11 @@ int32_t gtgpu_count_dev(gtgpu_index* index, uint64_t n, const uint32_t* d_chr, c
 /* Fused count → device-wide exclusive scan → emit in ONE pass over the queries (the device-resident core of
  * gtgpu_find / gtgpu_tokenize_files).  d_out_ids has room for ids_capacity ids; d_out_offsets (n+1 u64, per query)
  * and d_out_file_token_offsets (n_files+1 u64, RAW: before the [unk] rule; needs d_file_offsets) may each be NULL.
- * *d_out_total (device u64) receives the number of ids the call produces; when it exceeds ids_capacity the
- * surplus is not written (the host entry points then re-run with an exact buffer). */
+ * *d_out_total (device u64) receives the number of ids the call produces; when it exceeds ids_capacity the first
+ * ids_capacity ids are written exactly and the surplus is not written, while the total and both offset arrays are still
+ * complete (the host entry points then re-run with an exact buffer).  d_out_ids may be NULL when ids_capacity is 0.
+ * The kernel's overflow flag (a tile whose ids do not fit its 32-bit sums, or a running total of 2^55 or more) is not
+ * reported here; the host entry points fail with GTGPU_ERR_UNSUPPORTED on it. */
 int32_t gtgpu_find_dev(gtgpu_index* index, uint64_t n, const uint32_t* d_chr, const uint32_t* d_start,
                        const uint32_t* d_end, int32_t min_overlap, uint64_t n_files, const uint64_t* d_file_offsets,
                        uint32_t* d_out_ids, uint64_t ids_capacity, uint64_t* d_out_offsets,
