@@ -442,7 +442,8 @@ class Tokenizer:
 
 def tokenize_fragment_file(path, tokenizer: Tokenizer, device_parse: bool = False) -> dict:
     """gtars.tokenizers.tokenize_fragment_file (gtars-tokenizers/src/utils/fragments.rs:61-82): barcode -> token ids.
-    device_parse=True also parses the text and numbers the barcodes on the device (gtgpu_tokenize_fragments_text)."""
+    device_parse=True also parses the text and numbers the barcodes on the device (gtgpu_tokenize_fragments_file / _gz),
+    for a file of any size."""
     fn = lib().gth_tokenizer_fragments_device if device_parse else lib().gth_tokenizer_fragments
     return dict(_take_lists(fn(tokenizer._h, os.fsencode(path)), named=True))
 

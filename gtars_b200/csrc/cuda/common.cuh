@@ -369,26 +369,46 @@ struct DevMem {
     void swap(DevMem& o) { std::swap(ptr, o.ptr); std::swap(cap, o.cap); }
     uint32_t* u32() const { return static_cast<uint32_t*>(ptr); }
 };
-// Barcodes of one fragment file over all its windows (scoring): dense ids in first-appearance order, only barcodes seen on a
-// chromosome of the name table kept.  chr / start / end / bc hold every fragment of the file once finish() has run.
+// Barcodes of one fragment file over all its windows: dense ids in first-appearance order among the kept barcodes.  keep_all
+// (tokenization) keeps every barcode; otherwise (scoring) only those seen on a chromosome of the name table are kept.
+// record_spans keeps each barcode's first byte offset in the file for finish()'s spans.  who / array_entry name the caller and
+// its array entry point in error messages.  chr / start / end / bc hold every fragment of the file once finish() has run.
 struct FragBarcodeTable {
-    DevMem chr, start, end, fidx, known, hlen, bc;
+    const bool keep_all, record_spans;
+    const std::string who, array_entry;
+    DevMem chr, start, end, fidx, known, hlen, first_byte, bc;
     DevMem keys, first, soff, arena;
     uint64_t n = 0, distinct = 0, cap = 0, used = 0;
-    int32_t add_window(gtgpu_ctx* ctx, const char* d_text, const FragParse& fp, uint32_t n_names);
-    // *out_names: the kept barcodes' bytes back to back (elem_size 1); *out_name_offsets: n_kept + 1 u64 offsets into them
-    int32_t finish(gtgpu_ctx* ctx, uint32_t* n_kept, BufPtr* out_names, BufPtr* out_name_offsets);
+    FragBarcodeTable(bool keep_all_, bool record_spans_, std::string who_, std::string array_entry_)
+        : keep_all(keep_all_), record_spans(record_spans_), who(std::move(who_)), array_entry(std::move(array_entry_)) {}
+    // byte0: the window's offset in the file
+    int32_t add_window(gtgpu_ctx* ctx, const char* d_text, uint64_t byte0, const FragParse& fp, uint32_t n_names);
+    // With out_spans (needs record_spans): n_kept (first byte, length) u32 pairs, and out_names / out_name_offsets are untouched.
+    // Otherwise *out_names: the kept barcodes' bytes back to back (elem_size 1); *out_name_offsets: n_kept + 1 u64 offsets into them.
+    int32_t finish(gtgpu_ctx* ctx, uint32_t* n_kept, BufPtr* out_names, BufPtr* out_name_offsets, BufPtr* out_spans = nullptr);
 };
+// A fragment text of any size in windows that end right after a '\n' (about GTGPU_INGEST_WINDOW bytes, default 2 GiB).  fn gets
+// each window's device bytes, its size, its byte offset in the file and the file-wide index of its first line, and returns
+// the window's line count.  Exactly one of host_text (staged through pinned memory) / dev_text (read in place) is given.
+using WindowFn = std::function<int32_t(const char* d_window, uint64_t n_bytes, uint64_t byte0, uint64_t first_line, uint32_t* n_lines)>;
+int32_t for_each_window(gtgpu_ctx* ctx, const char* host_text, const char* dev_text, uint64_t n_bytes, const std::string& who,
+                        const WindowFn& fn);
 // inflate.cu: H2D of gzip members + inflate; the text stays in scratch SC_GZ_OUT
 int32_t check_members(uint64_t n_members, const uint8_t* gz, const uint64_t* member_offsets, const char* who);
 int32_t gunzip_locked(gtgpu_ctx* ctx, uint64_t n_members, const uint8_t* gz, const uint64_t* member_offsets,
                       uint64_t* out_member_offsets, uint8_t** d_text, uint64_t* n_text);
+// gunzip_locked for a text parsed in windows afterwards: a text that does not fit in device memory is reported as such
+int32_t inflate_whole_locked(gtgpu_ctx* ctx, uint64_t n_members, const uint8_t* gz, const uint64_t* member_offsets, const std::string& who,
+                             uint8_t** d_text, uint64_t* n_text);
 // The text is host_text (copied to the device here) or dev_text (already there, e.g. inflated): exactly one is non-null.
 int32_t tokenize_bed_locked(gtgpu_index* ix, const char* host_text, const char* dev_text, uint64_t n_bytes, uint32_t n_names,
                             const char* names, const uint32_t* name_offsets, uint32_t unk_id, gtgpu_buf** out_ids);
-int32_t tokenize_fragments_text_locked(gtgpu_index* ix, const char* host_text, const char* dev_text, uint64_t n_bytes, uint32_t n_names,
-                                       const char* names, const uint32_t* name_offsets, uint32_t unk_id, uint32_t* out_n_barcodes,
-                                       BufPtr* out_barcode_spans, BufPtr* out_barcode_offsets, BufPtr* out_ids);
+// Fragment tokenization of a text of any size; barcodes as names (out_names, out_name_offsets) or, with out_spans, as u32
+// (first byte, length) spans into the text (the text must then be < 4 GiB).
+int32_t tokenize_fragments_file_locked(gtgpu_index* ix, const char* host_text, const char* dev_text, uint64_t n_bytes, uint32_t n_names,
+                                       const char* names, const uint32_t* name_offsets, uint32_t unk_id, const std::string& who,
+                                       uint32_t* out_n_barcodes, BufPtr* out_names, BufPtr* out_name_offsets, BufPtr* out_spans,
+                                       BufPtr* out_barcode_offsets, BufPtr* out_ids);
 
 // groups (api.cu, comm.cu, igd.cu)
 int32_t for_each_device(size_t n_devices, const std::function<int32_t(size_t)>& fn);

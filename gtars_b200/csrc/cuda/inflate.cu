@@ -612,6 +612,16 @@ int32_t gunzip_locked(gtgpu_ctx* ctx, uint64_t n_members, const uint8_t* gz, con
     return gunzip_device(ctx, n_members, d_gz, d_mo, d_oo, d_out, d_status, h_status);
 }
 
+// gzip members -> device text (SC_GZ_OUT); a text that does not fit in device memory is reported as such
+int32_t inflate_whole_locked(gtgpu_ctx* ctx, uint64_t n_members, const uint8_t* gz, const uint64_t* member_offsets, const std::string& who,
+                             uint8_t** d_text, uint64_t* n_text) {
+    const int32_t s = gunzip_locked(ctx, n_members, gz, member_offsets, nullptr, d_text, n_text);
+    if (s == GTGPU_ERR_NOMEM)
+        return fail(s, who + ": the inflated text does not fit in device memory (gzip input is inflated whole before it is parsed): " +
+                           gtgpu_last_error());
+    return s;
+}
+
 int32_t check_members(uint64_t n_members, const uint8_t* gz, const uint64_t* member_offsets, const char* who) {
     if (n_members && (!gz || !member_offsets)) return fail(GTGPU_ERR_INVALID, std::string(who) + ": null argument");
     for (uint64_t k = 0; k < n_members; ++k)
@@ -656,7 +666,7 @@ extern "C" int32_t gtgpu_tokenize_bed_gz(gtgpu_index* ix, uint64_t n_members, co
 } GT_CATCH
 
 // gtgpu_tokenize_fragments_text on gzip members (a bgzip'ed fragment file: thousands of members).  *out_text returns the
-// inflated text as well: the barcode spans index into it.
+// inflated text as well: the barcode spans index into it.  Errors carry the text form's name and messages.
 extern "C" int32_t gtgpu_tokenize_fragments_gz(gtgpu_index* ix, uint64_t n_members, const uint8_t* gz, const uint64_t* member_offsets,
                                                uint32_t n_names, const char* names, const uint32_t* name_offsets, uint32_t unk_id,
                                                uint32_t* out_n_barcodes, gtgpu_buf** out_barcode_spans,
@@ -671,13 +681,14 @@ extern "C" int32_t gtgpu_tokenize_fragments_gz(gtgpu_index* ix, uint64_t n_membe
     uint8_t* d_text = nullptr;
     uint64_t n_text = 0;
     GT_TRY(gunzip_locked(ctx, n_members, gz, member_offsets, nullptr, &d_text, &n_text));
+    if (n_text >= 0xFFFFFFF0ull) return fail(GTGPU_ERR_UNSUPPORTED, "tokenize_fragments_text: at most 4 GiB of text per call");
     BufPtr text, spans, offs, ids;  // the text's copy on copy_out overlaps the parse
     int32_t s = buf_from_device(ctx, d_text, n_text, 1, ctx->copy_out, &text);
     if (s == GTGPU_ERR_CUDA) return fail(s, "tokenize_fragments_gz: D2H of the text failed");
     GT_TRY(s);
     try {
-        s = tokenize_fragments_text_locked(ix, nullptr, (const char*)d_text, n_text, n_names, names, name_offsets, unk_id, out_n_barcodes,
-                                           &spans, &offs, &ids);
+        s = tokenize_fragments_file_locked(ix, nullptr, (const char*)d_text, n_text, n_names, names, name_offsets, unk_id,
+                                           "tokenize_fragments_text", out_n_barcodes, nullptr, nullptr, &spans, &offs, &ids);
     } catch (...) {
         cudaStreamSynchronize(ctx->copy_out);  // the text's copy ends before its block goes back to the cache
         throw;
@@ -691,5 +702,31 @@ extern "C" int32_t gtgpu_tokenize_fragments_gz(gtgpu_index* ix, uint64_t n_membe
     *out_barcode_offsets = offs.release();
     *out_ids = ids.release();
     *out_text = text.release();
+    return GTGPU_OK;
+} GT_CATCH
+
+// gtgpu_tokenize_fragments_file on gzip members: inflated whole into device memory, then tokenized in windows where it is.
+extern "C" int32_t gtgpu_tokenize_fragments_file_gz(gtgpu_index* ix, uint64_t n_members, const uint8_t* gz, const uint64_t* member_offsets,
+                                                    uint32_t n_names, const char* names, const uint32_t* name_offsets, uint32_t unk_id,
+                                                    uint32_t* out_n_barcodes, gtgpu_buf** out_barcode_names,
+                                                    gtgpu_buf** out_barcode_name_offsets, gtgpu_buf** out_barcode_offsets,
+                                                    gtgpu_buf** out_ids) try {
+    if (!ix || !out_n_barcodes || !out_barcode_names || !out_barcode_name_offsets || !out_barcode_offsets || !out_ids ||
+        (n_names && (!names || !name_offsets)))
+        return fail(GTGPU_ERR_INVALID, "tokenize_fragments_file_gz: null argument");
+    GT_TRY(check_members(n_members, gz, member_offsets, "tokenize_fragments_file_gz"));
+    gtgpu_ctx* ctx = ix->ctx;
+    std::lock_guard<std::mutex> lk(ctx->mu);
+    GT_CUDA(cudaSetDevice(ctx->device));
+    uint8_t* d_text = nullptr;
+    uint64_t n_text = 0;
+    GT_TRY(inflate_whole_locked(ctx, n_members, gz, member_offsets, "tokenize_fragments_file_gz", &d_text, &n_text));
+    BufPtr nm, no, offs, ids;
+    GT_TRY(tokenize_fragments_file_locked(ix, nullptr, (const char*)d_text, n_text, n_names, names, name_offsets, unk_id,
+                                          "tokenize_fragments_file_gz", out_n_barcodes, &nm, &no, nullptr, &offs, &ids));
+    *out_barcode_names = nm.release();
+    *out_barcode_name_offsets = no.release();
+    *out_barcode_offsets = offs.release();
+    *out_ids = ids.release();
     return GTGPU_OK;
 } GT_CATCH

@@ -14,9 +14,11 @@
 // regions ever existing on the host.  Chromosome names that are not in the table map to GTGPU_UNKNOWN_CHROM and sort
 // after every known name (the reference sorts them by their own strings; they produce no output either way).
 #include <algorithm>
+#include <cstdlib>
 #include <cstring>
 #include <numeric>
 #include <string>
+#include <thread>
 #include <vector>
 
 #include "common.cuh"
@@ -300,43 +302,12 @@ __global__ void ingest_barcode_insert_kernel(uint32_t n, const unsigned long lon
     }
 }
 
-// 1 for the fragment that is the first appearance of its barcode; also checks that a fragment's barcode bytes equal
-// those of the first appearance (two different barcodes with one 64-bit hash would otherwise be merged silently).
-__global__ void ingest_barcode_heads_kernel(uint32_t n, const char* __restrict__ text, const uint32_t* __restrict__ slot_of,
-                                            const uint32_t* __restrict__ first, const uint32_t* __restrict__ bo,
-                                            const uint32_t* __restrict__ bl, uint32_t* __restrict__ head, uint32_t* __restrict__ collision) {
-    const uint32_t stride = gridDim.x * blockDim.x;
-    for (uint32_t k = blockIdx.x * blockDim.x + threadIdx.x; k < n; k += stride) {
-        const uint32_t f = first[slot_of[k]];
-        head[k] = f == k;
-        if (f != k) {
-            bool same = bl[f] == bl[k];
-            for (uint32_t i = 0; same && i < bl[k]; ++i) same = text[bo[f] + i] == text[bo[k] + i];
-            if (!same) *collision = 1;
-        }
-    }
-}
-
-__global__ void ingest_barcode_ids_kernel(uint32_t n, const uint32_t* __restrict__ slot_of, const uint32_t* __restrict__ first,
-                                          const uint32_t* __restrict__ rank, const uint32_t* __restrict__ bo, const uint32_t* __restrict__ bl,
-                                          uint32_t* __restrict__ bc_id, uint32_t* __restrict__ spans) {
-    const uint32_t stride = gridDim.x * blockDim.x;
-    for (uint32_t k = blockIdx.x * blockDim.x + threadIdx.x; k < n; k += stride) {
-        const uint32_t f = first[slot_of[k]];
-        const uint32_t id = rank[f];  // first appearances are numbered in file order by the scan over `head`
-        bc_id[k] = id;
-        if (f == k) {
-            spans[2 * id] = bo[k];
-            spans[2 * id + 1] = bl[k];
-        }
-    }
-}
-
-// ---- the barcode table of the scoring entry points: one table over all windows of a file -----------------------------------
+// ---- the barcode table of the fragment-text entry points: one table over all windows of a file ------------------------------
 // A window's fragments are numbered file-wide (base + k), so a slot's first-appearance index is the file-wide index of the
 // barcode's first fragment.  Per fragment the table keeps fidx (that index), per barcode (at its first fragment g) hlen[g]
-// (its byte length) and known[g] (seen on a chromosome of the name table); the bytes go to an arena in the window that
-// first sees the barcode, in first-appearance order, because the text of a plain-text window leaves the device with it.
+// (its byte length), known[g] (seen on a chromosome of the name table) and, when asked for, first_byte[g] (the file offset of
+// its first occurrence); the bytes go to an arena in the window that first sees the barcode, in first-appearance order,
+// because the text of a plain-text window leaves the device with it.
 __global__ void ingest_barcode_rehash_kernel(uint64_t old_cap, const unsigned long long* __restrict__ okeys,
                                              const uint32_t* __restrict__ ofirst, const unsigned long long* __restrict__ osoff,
                                              uint32_t mask, unsigned long long* __restrict__ keys, uint32_t* __restrict__ first,
@@ -371,13 +342,15 @@ __global__ void ingest_barcode_window_heads_kernel(uint32_t n, uint32_t base, co
 __global__ void ingest_barcode_claim_kernel(uint32_t n, uint32_t base, const char* __restrict__ text, const uint32_t* __restrict__ slot_of,
                                             const uint32_t* __restrict__ fidx, const uint32_t* __restrict__ bo,
                                             const uint32_t* __restrict__ bl, const uint32_t* __restrict__ wpos, uint64_t used,
-                                            char* __restrict__ arena, unsigned long long* __restrict__ soff) {
+                                            char* __restrict__ arena, unsigned long long* __restrict__ soff, uint64_t byte0,
+                                            unsigned long long* __restrict__ first_byte) {
     const uint32_t stride = gridDim.x * blockDim.x;
     for (uint32_t k = blockIdx.x * blockDim.x + threadIdx.x; k < n; k += stride) {
         if (fidx[base + k] != base + k) continue;
         const uint64_t p = used + wpos[k];
         for (uint32_t i = 0; i < bl[k]; ++i) arena[p + i] = text[bo[k] + i];
         soff[slot_of[k]] = p;
+        if (first_byte) first_byte[base + k] = byte0 + bo[k];
     }
 }
 
@@ -398,14 +371,15 @@ __global__ void ingest_barcode_check_kernel(uint32_t n, uint32_t base, const cha
     }
 }
 
-// after the last window: a barcode is kept when it was seen on a known chromosome; alen / klen are the byte lengths of every
-// first appearance / of the kept ones (u64 for the scans)
-__global__ void ingest_barcode_keep_kernel(uint64_t n, const uint32_t* __restrict__ fidx, const uint32_t* __restrict__ known,
-                                           const uint32_t* __restrict__ hlen, uint32_t* __restrict__ keep,
-                                           unsigned long long* __restrict__ alen, unsigned long long* __restrict__ klen) {
+// after the last window: a barcode is kept when keep_all is set or it was seen on a known chromosome; alen / klen are the byte
+// lengths of every first appearance / of the kept ones (u64 for the scans)
+__global__ void ingest_barcode_keep_kernel(uint64_t n, uint32_t keep_all, const uint32_t* __restrict__ fidx,
+                                           const uint32_t* __restrict__ known, const uint32_t* __restrict__ hlen,
+                                           uint32_t* __restrict__ keep, unsigned long long* __restrict__ alen,
+                                           unsigned long long* __restrict__ klen) {
     const uint64_t stride = (uint64_t)gridDim.x * blockDim.x;
     for (uint64_t g = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x; g < n; g += stride) {
-        const bool kp = fidx[g] == g && known[g];
+        const bool kp = fidx[g] == g && (keep_all || known[g]);
         keep[g] = kp;
         alen[g] = hlen[g];
         klen[g] = kp ? hlen[g] : 0u;
@@ -413,19 +387,27 @@ __global__ void ingest_barcode_keep_kernel(uint64_t n, const uint32_t* __restric
 }
 
 // dense ids in first-appearance order among the kept barcodes; a fragment of a dropped barcode lies on an unknown chromosome
-// (it has no hit), so any valid id serves it.  The kept names are gathered from the arena in id order.
+// (it has no hit), so any valid id serves it.  The kept names are gathered from the arena in id order (blob != nullptr), or
+// their (first byte, length) spans are written in id order (spans != nullptr).
 __global__ void ingest_barcode_final_kernel(uint64_t n, const uint32_t* __restrict__ fidx, const uint32_t* __restrict__ keep,
                                             const uint32_t* __restrict__ rank, const unsigned long long* __restrict__ aoff,
                                             const unsigned long long* __restrict__ boff, const uint32_t* __restrict__ hlen,
                                             const char* __restrict__ arena, char* __restrict__ blob,
-                                            unsigned long long* __restrict__ name_off, uint32_t* __restrict__ bc) {
+                                            unsigned long long* __restrict__ name_off, const unsigned long long* __restrict__ first_byte,
+                                            uint32_t* __restrict__ spans, uint32_t* __restrict__ bc) {
     const uint64_t stride = (uint64_t)gridDim.x * blockDim.x;
     for (uint64_t g = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x; g < n; g += stride) {
         const uint32_t f = fidx[g];
         bc[g] = keep[f] ? rank[f] : 0u;
         if (keep[g]) {
-            for (uint32_t i = 0; i < hlen[g]; ++i) blob[boff[g] + i] = arena[aoff[g] + i];
-            name_off[rank[g]] = boff[g];
+            if (blob) {
+                for (uint32_t i = 0; i < hlen[g]; ++i) blob[boff[g] + i] = arena[aoff[g] + i];
+                name_off[rank[g]] = boff[g];
+            }
+            if (spans) {
+                spans[2 * (uint64_t)rank[g]] = (uint32_t)first_byte[g];
+                spans[2 * (uint64_t)rank[g] + 1] = hlen[g];
+            }
         }
     }
 }
@@ -549,6 +531,126 @@ int32_t parse_fragments_locked(gtgpu_ctx* ctx, const char* d_text, uint64_t n_by
     out->free2 = p_chr;
     out->tmp = d_tmp;
     out->flags = d_flags;
+    return GTGPU_OK;
+}
+
+// ---- fragment text of any size, window by window (scoring and tokenization) --------------------------------------------------
+// The text is parsed in windows (the parse kernels address a window with u32 positions): a window ends right after the first
+// '\n' at or past its nominal size, so it holds whole lines, and a window's local line index plus the lines of the windows
+// before it is the file-wide index the host parser reports.  Plain text is copied window by window (the copy of window k+1,
+// through pinned staging on the copy stream, overlaps the kernels of window k); device text (e.g. inflated gzip members) is
+// read where it is.
+
+// GTGPU_INGEST_WINDOW=<bytes>, read per call: nominal window size (results never depend on it)
+static uint64_t ingest_window_bytes() {
+    uint64_t w = 2ull << 30;
+    if (const char* env = getenv("GTGPU_INGEST_WINDOW")) {
+        const uint64_t v = strtoull(env, nullptr, 10);
+        if (v) w = v;
+    }
+    return std::min<uint64_t>(w, 3ull << 30);
+}
+
+struct StagingScope {  // pinned staging blocks and their events, returned to the ctx when the call ends
+    gtgpu_ctx* ctx;
+    PinnedBlock pin[2];
+    cudaEvent_t ev[2] = {nullptr, nullptr};
+    bool used[2] = {false, false};
+    explicit StagingScope(gtgpu_ctx* c) : ctx(c) {}
+    ~StagingScope() {
+        cudaStreamSynchronize(ctx->copy_in);
+        for (int b = 0; b < 2; ++b) {
+            if (ev[b]) cudaEventDestroy(ev[b]);
+            ctx->pinned_put(pin[b]);
+        }
+    }
+};
+
+int32_t for_each_window(gtgpu_ctx* ctx, const char* host_text, const char* dev_text, uint64_t n_bytes, const std::string& who,
+                        const WindowFn& fn) {
+    cudaStream_t st = ctx->stream;
+    const uint64_t W = ingest_window_bytes();
+    std::vector<uint64_t> cut{0};  // window w = [cut[w], cut[w + 1])
+    while (cut.back() < n_bytes) {
+        const uint64_t a = cut.back();
+        uint64_t b = n_bytes;
+        if (n_bytes - a > W) {
+            const uint64_t p = a + W - 1;
+            if (host_text) {
+                const void* q = memchr(host_text + p, '\n', n_bytes - p);
+                if (q) b = (uint64_t)((const char*)q - host_text) + 1;
+            } else {
+                char piece[4096];
+                for (uint64_t q = p; q < n_bytes && b == n_bytes; q += sizeof piece) {
+                    const uint64_t len = std::min<uint64_t>(sizeof piece, n_bytes - q);
+                    GT_CUDA(cudaMemcpyAsync(piece, dev_text + q, len, cudaMemcpyDeviceToHost, st));
+                    GT_CUDA(cudaStreamSynchronize(st));
+                    const void* nl = memchr(piece, '\n', len);
+                    if (nl) b = q + (uint64_t)((const char*)nl - piece) + 1;
+                }
+            }
+        }
+        if (b - a >= 0xFFFFFFF0ull) return fail(GTGPU_ERR_UNSUPPORTED, who + ": a line of 4 GiB or more");
+        cut.push_back(b);
+    }
+    const size_t n_win = cut.size() - 1;
+    uint64_t max_win = 0;
+    for (size_t w = 0; w < n_win; ++w) max_win = std::max(max_win, cut[w + 1] - cut[w]);
+    uint64_t first_line = 0;
+    uint32_t n_lines = 0;
+    if (dev_text) {
+        char* d_copy = nullptr;  // windows that do not start 16-byte aligned are moved to aligned scratch (the newline scan loads 16 B)
+        for (size_t w = 0; w < n_win; ++w) {
+            const char* d = dev_text + cut[w];
+            if (reinterpret_cast<uintptr_t>(d) & 15) {
+                if (!d_copy) GT_TRY(ctx->scratch_get(SC_WIN_A, max_win + 64, (void**)&d_copy));
+                GT_CUDA(cudaMemcpyAsync(d_copy, d, cut[w + 1] - cut[w], cudaMemcpyDeviceToDevice, st));
+                d = d_copy;
+            }
+            GT_TRY(fn(d, cut[w + 1] - cut[w], cut[w], first_line, &n_lines));
+            first_line += n_lines;
+        }
+        return GTGPU_OK;
+    }
+    char* dbuf[2] = {nullptr, nullptr};
+    GT_TRY(ctx->scratch_get(SC_WIN_A, max_win + 64, (void**)&dbuf[0]));
+    if (n_win > 1) GT_TRY(ctx->scratch_get(SC_WIN_B, max_win + 64, (void**)&dbuf[1]));
+    StagingScope sg(ctx);
+    const uint64_t piece = std::min<uint64_t>(max_win, 64ull << 20);
+    for (int b = 0; b < 2; ++b) {
+        GT_TRY(ctx->pinned_get(piece, &sg.pin[b]));
+        GT_CUDA(cudaEventCreateWithFlags(&sg.ev[b], cudaEventDisableTiming));
+    }
+    // window w -> dbuf[w % 2] through the two pinned pieces; runs on a helper thread while the kernels of window w - 1 run
+    std::string stage_err;
+    auto stage = [&](size_t w) -> int32_t {
+        if (cudaSetDevice(ctx->device) != cudaSuccess) return GTGPU_ERR_CUDA;
+        cudaError_t e = cudaSuccess;
+        uint64_t j = 0;
+        for (uint64_t off = cut[w]; off < cut[w + 1] && e == cudaSuccess; off += piece, ++j) {
+            const int b = (int)(j & 1);
+            const uint64_t len = std::min(piece, cut[w + 1] - off);
+            if (sg.used[b]) e = cudaEventSynchronize(sg.ev[b]);
+            if (e != cudaSuccess) break;
+            memcpy(sg.pin[b].ptr, host_text + off, len);
+            e = cudaMemcpyAsync(dbuf[w & 1] + (off - cut[w]), sg.pin[b].ptr, len, cudaMemcpyHostToDevice, ctx->copy_in);
+            if (e == cudaSuccess) e = cudaEventRecord(sg.ev[b], ctx->copy_in);
+            sg.used[b] = true;
+        }
+        if (e == cudaSuccess) e = cudaStreamSynchronize(ctx->copy_in);
+        if (e != cudaSuccess) stage_err = std::string("H2D of the text: ") + cudaGetErrorString(e);
+        return e == cudaSuccess ? GTGPU_OK : GTGPU_ERR_CUDA;
+    };
+    int32_t s_next = stage(0);
+    for (size_t w = 0; w < n_win && s_next == GTGPU_OK; ++w) {
+        std::thread helper;
+        if (w + 1 < n_win) helper = std::thread([&, w] { s_next = stage(w + 1); });
+        const int32_t s = fn(dbuf[w & 1], cut[w + 1] - cut[w], cut[w], first_line, &n_lines);
+        if (helper.joinable()) helper.join();
+        if (s != GTGPU_OK) return s;
+        first_line += n_lines;
+    }
+    if (s_next != GTGPU_OK) return fail(s_next, who + ": " + stage_err);
     return GTGPU_OK;
 }
 
@@ -713,13 +815,14 @@ DevMem::~DevMem() {
     if (ptr) cudaFree(ptr);
 }
 
-int32_t FragBarcodeTable::add_window(gtgpu_ctx* ctx, const char* d_text, const FragParse& fp, uint32_t n_names) {
+int32_t FragBarcodeTable::add_window(gtgpu_ctx* ctx, const char* d_text, uint64_t byte0, const FragParse& fp, uint32_t n_names) {
     const uint32_t nw = fp.n;
     if (nw == 0) return GTGPU_OK;
     cudaStream_t st = ctx->stream;
     const uint32_t base = (uint32_t)n;
     const size_t need = (size_t)(n + nw) * 4, have = (size_t)n * 4;
     for (DevMem* m : {&chr, &start, &end, &fidx, &known, &hlen}) GT_TRY(m->reserve(need, have, st));
+    if (record_spans) GT_TRY(first_byte.reserve(need * 2, have * 2, st));
     GT_CUDA(cudaMemcpyAsync(chr.u32() + base, fp.chr, (size_t)nw * 4, cudaMemcpyDeviceToDevice, st));
     GT_CUDA(cudaMemcpyAsync(start.u32() + base, fp.start, (size_t)nw * 4, cudaMemcpyDeviceToDevice, st));
     GT_CUDA(cudaMemcpyAsync(end.u32() + base, fp.end, (size_t)nw * 4, cudaMemcpyDeviceToDevice, st));
@@ -762,25 +865,27 @@ int32_t FragBarcodeTable::add_window(gtgpu_ctx* ctx, const char* d_text, const F
     const uint64_t bytes = (uint64_t)tail[0] + tail[1];
     GT_TRY(arena.reserve(used + bytes + 1, used, st));
     ingest_barcode_claim_kernel<<<igrid(ctx, nw), 256, 0, st>>>(nw, base, d_text, slot_of, fidx.u32(), fp.bo, fp.bl, wpos, used,
-                                                                (char*)arena.ptr, (unsigned long long*)soff.ptr);
+                                                                (char*)arena.ptr, (unsigned long long*)soff.ptr, byte0,
+                                                                (unsigned long long*)first_byte.ptr);
     ingest_barcode_check_kernel<<<igrid(ctx, nw), 256, 0, st>>>(nw, base, d_text, slot_of, fidx.u32(), fp.bo, fp.bl, hlen.u32(),
                                                                 (const char*)arena.ptr, (const unsigned long long*)soff.ptr, fp.flags + 1);
     ctx->launches += 2;
     uint32_t collision = 0;
     GT_CUDA(cudaMemcpyAsync(&collision, fp.flags + 1, 4, cudaMemcpyDeviceToHost, st));
     GT_CUDA(cudaStreamSynchronize(st));  // the window's text may be overwritten after this
-    if (collision) return fail(GTGPU_ERR_UNSUPPORTED, "two barcodes share a 64-bit hash; use gtgpu_score_barcodes");
+    if (collision) return fail(GTGPU_ERR_UNSUPPORTED, who + ": two barcodes share a 64-bit hash; use " + array_entry);
     used += bytes;
     distinct += tail[2];
     n += nw;
     return GTGPU_OK;
 }
 
-int32_t FragBarcodeTable::finish(gtgpu_ctx* ctx, uint32_t* n_kept, BufPtr* out_names, BufPtr* out_name_offsets) {
+int32_t FragBarcodeTable::finish(gtgpu_ctx* ctx, uint32_t* n_kept, BufPtr* out_names, BufPtr* out_name_offsets, BufPtr* out_spans) {
     cudaStream_t st = ctx->stream;
     uint64_t kept = 0, blob_bytes = 0;
     char* d_blob = nullptr;
     unsigned long long* d_noff = nullptr;
+    uint32_t* d_spans = nullptr;
     if (n) {
         uint32_t *d_keep, *d_rank;
         unsigned long long *d_alen, *d_klen, *d_aoff, *d_boff;
@@ -793,7 +898,8 @@ int32_t FragBarcodeTable::finish(gtgpu_ctx* ctx, uint32_t* n_kept, BufPtr* out_n
         GT_TRY(ctx->scratch_get(SC_ING_4, n * 8, (void**)&d_boff));
         GT_TRY(ctx->scratch_get(SC_IN3_START, exclusive_scan_temp_bytes(n, 8), &d_tmp));
         GT_TRY(bc.reserve(n * 4, 0, st));
-        ingest_barcode_keep_kernel<<<igrid(ctx, n), 256, 0, st>>>(n, fidx.u32(), known.u32(), hlen.u32(), d_keep, d_alen, d_klen);
+        ingest_barcode_keep_kernel<<<igrid(ctx, n), 256, 0, st>>>(n, keep_all, fidx.u32(), known.u32(), hlen.u32(), d_keep, d_alen,
+                                                                  d_klen);
         ctx->launches++;
         GT_TRY(exclusive_scan<uint32_t>(ctx, d_keep, d_rank, n, d_tmp));
         GT_TRY(exclusive_scan<unsigned long long>(ctx, d_alen, d_aoff, n, d_tmp));
@@ -807,29 +913,79 @@ int32_t FragBarcodeTable::finish(gtgpu_ctx* ctx, uint32_t* n_kept, BufPtr* out_n
         GT_CUDA(cudaStreamSynchronize(st));
         kept = (uint64_t)t32[0] + t32[1];
         blob_bytes = t64[0] + t64[1];
-        GT_TRY(ctx->scratch_get(SC_ING_6, blob_bytes + 1, (void**)&d_blob));
-        GT_TRY(ctx->scratch_get(SC_ING_7, (kept + 1) * 8, (void**)&d_noff));
+        if (out_spans) {
+            GT_TRY(ctx->scratch_get(SC_FILE_OFFS, kept * 8 + 8, (void**)&d_spans));
+        } else {
+            GT_TRY(ctx->scratch_get(SC_ING_6, blob_bytes + 1, (void**)&d_blob));
+            GT_TRY(ctx->scratch_get(SC_ING_7, (kept + 1) * 8, (void**)&d_noff));
+        }
         ingest_barcode_final_kernel<<<igrid(ctx, n), 256, 0, st>>>(n, fidx.u32(), d_keep, d_rank, d_aoff, d_boff, hlen.u32(),
-                                                                   (const char*)arena.ptr, d_blob, d_noff, bc.u32());
+                                                                   (const char*)arena.ptr, d_blob, d_noff,
+                                                                   (const unsigned long long*)first_byte.ptr, d_spans, bc.u32());
         ctx->launches++;
         GT_CUDA(cudaGetLastError());
     }
+    *n_kept = (uint32_t)kept;
+    if (out_spans) {
+        BufPtr spans;
+        int32_t s = buf_from_device(ctx, d_spans, kept * 2, 4, st, &spans);
+        if (s == GTGPU_ERR_CUDA) return fail(s, who + ": D2H of the barcode spans failed");
+        GT_TRY(s);
+        if (cudaStreamSynchronize(st) != cudaSuccess) return fail(GTGPU_ERR_CUDA, who + ": D2H of the barcode spans failed");
+        *out_spans = std::move(spans);
+        return GTGPU_OK;
+    }
     BufPtr names, offsets;
     int32_t s = buf_from_device(ctx, d_blob, blob_bytes, 1, st, &names);
-    if (s == GTGPU_ERR_CUDA) return fail(s, "score_barcodes_text: D2H of the barcode names failed");
+    if (s == GTGPU_ERR_CUDA) return fail(s, who + ": D2H of the barcode names failed");
     GT_TRY(s);
     s = buf_new(ctx, kept + 1, 8, &offsets);  // the last offset is written on the host
     if (s == GTGPU_OK && kept && cudaMemcpyAsync(offsets->block.ptr, d_noff, kept * 8, cudaMemcpyDeviceToHost, st) != cudaSuccess)
-        s = fail(GTGPU_ERR_CUDA, "score_barcodes_text: D2H of the barcode name offsets failed");
-    if (s == GTGPU_OK && cudaStreamSynchronize(st) != cudaSuccess) s = fail(GTGPU_ERR_CUDA, "score_barcodes_text: D2H failed");
+        s = fail(GTGPU_ERR_CUDA, who + ": D2H of the barcode name offsets failed");
+    if (s == GTGPU_OK && cudaStreamSynchronize(st) != cudaSuccess) s = fail(GTGPU_ERR_CUDA, who + ": D2H failed");
     if (s != GTGPU_OK) {
         cudaStreamSynchronize(st);  // the names' copy may still run
         return s;
     }
     reinterpret_cast<uint64_t*>(offsets->block.ptr)[kept] = blob_bytes;
-    *n_kept = (uint32_t)kept;
     *out_names = std::move(names);
     *out_name_offsets = std::move(offsets);
+    return GTGPU_OK;
+}
+
+// tokenize_fragment_file (fragments.rs:61-82) from a fragment file's text of any size: every window is parsed and its barcodes
+// go into one FragBarcodeTable that keeps every barcode; after the last window the fragment tokenizer core runs once over the
+// accumulated fragments and their dense barcode ids.  With out_spans the barcodes come back as u32 (first byte, length) spans
+// into the text, else as names + u64 name offsets.  The caller holds ctx->mu.
+int32_t tokenize_fragments_file_locked(gtgpu_index* ix, const char* host_text, const char* dev_text, uint64_t n_bytes, uint32_t n_names,
+                                       const char* names, const uint32_t* name_offsets, uint32_t unk_id, const std::string& who,
+                                       uint32_t* out_n_barcodes, BufPtr* out_names, BufPtr* out_name_offsets, BufPtr* out_spans,
+                                       BufPtr* out_barcode_offsets, BufPtr* out_ids) {
+    gtgpu_ctx* ctx = ix->ctx;
+    FragBarcodeTable tab(true, out_spans != nullptr, who, "gtgpu_tokenize_fragments");
+    if (n_bytes) {
+        NameTable nt;
+        GT_TRY(upload_name_table(ctx, n_names, names, name_offsets, &nt));
+        GT_TRY(for_each_window(ctx, host_text, dev_text, n_bytes, who,
+                               [&](const char* d, uint64_t nb, uint64_t byte0, uint64_t line0, uint32_t* n_lines) -> int32_t {
+            FragParse fp;
+            GT_TRY(parse_fragments_locked(ctx, d, nb, nt, FRAG_TOKENIZE, &fp));
+            *n_lines = fp.n_lines;
+            if (fp.bad_line != 0xFFFFFFFFu)
+                return fail(GTGPU_ERR_INVALID, who + ": Invalid fragment file detected at line: " + std::to_string(line0 + fp.bad_line));
+            if (tab.n + fp.n > 0xFFFFFFFFull) return fail(GTGPU_ERR_UNSUPPORTED, who + ": more than 2^32 - 1 fragments in one file");
+            return tab.add_window(ctx, d, byte0, fp, n_names);
+        }));
+    }
+    uint32_t n_barcodes = 0;
+    BufPtr offs, ids;
+    GT_TRY(tab.finish(ctx, &n_barcodes, out_names, out_name_offsets, out_spans));
+    GT_TRY(buf_new(ctx, (uint64_t)n_barcodes + 1, 8, &offs));
+    GT_TRY(tokenize_fragments_core(ix, tab.n, tab.chr.u32(), tab.start.u32(), tab.end.u32(), tab.bc.u32(), n_barcodes, unk_id,
+                                   (uint64_t*)offs->block.ptr, &ids));
+    *out_n_barcodes = n_barcodes;
+    *out_barcode_offsets = std::move(offs);
+    *out_ids = std::move(ids);
     return GTGPU_OK;
 }
 
@@ -897,8 +1053,7 @@ int32_t gtgpu::tokenize_bed_locked(gtgpu_index* ix, const char* host_text, const
     return GTGPU_OK;
 }
 
-// tokenize_fragment_file (fragments.rs:61-82) from the file's text: parse on the device, barcodes -> dense ids in
-// first-appearance order through a device hash table, then the fragment tokenizer core.
+// tokenize_fragment_file (fragments.rs:61-82) from the file's text, < 4 GiB: the barcodes come back as u32 spans into the text.
 extern "C" int32_t gtgpu_tokenize_fragments_text(gtgpu_index* ix, const char* text, uint64_t n_bytes, uint32_t n_names,
                                                  const char* names, const uint32_t* name_offsets, uint32_t unk_id,
                                                  uint32_t* out_n_barcodes, gtgpu_buf** out_barcode_spans,
@@ -906,88 +1061,37 @@ extern "C" int32_t gtgpu_tokenize_fragments_text(gtgpu_index* ix, const char* te
     if (!ix || !out_n_barcodes || !out_barcode_spans || !out_barcode_offsets || !out_ids || (n_bytes && !text) ||
         (n_names && (!names || !name_offsets)))
         return fail(GTGPU_ERR_INVALID, "tokenize_fragments_text: null argument");
+    if (n_bytes >= 0xFFFFFFF0ull) return fail(GTGPU_ERR_UNSUPPORTED, "tokenize_fragments_text: at most 4 GiB of text per call");
     gtgpu_ctx* ctx = ix->ctx;
     std::lock_guard<std::mutex> lk(ctx->mu);
     GT_CUDA(cudaSetDevice(ctx->device));
     BufPtr spans, offs, ids;
-    GT_TRY(tokenize_fragments_text_locked(ix, text, nullptr, n_bytes, n_names, names, name_offsets, unk_id, out_n_barcodes, &spans,
-                                          &offs, &ids));
+    GT_TRY(tokenize_fragments_file_locked(ix, text, nullptr, n_bytes, n_names, names, name_offsets, unk_id, "tokenize_fragments_text",
+                                          out_n_barcodes, nullptr, nullptr, &spans, &offs, &ids));
     *out_barcode_spans = spans.release();
     *out_barcode_offsets = offs.release();
     *out_ids = ids.release();
     return GTGPU_OK;
 } GT_CATCH
 
-// the caller holds ctx->mu
-int32_t gtgpu::tokenize_fragments_text_locked(gtgpu_index* ix, const char* host_text, const char* dev_text, uint64_t n_bytes,
-                                              uint32_t n_names, const char* names, const uint32_t* name_offsets, uint32_t unk_id,
-                                              uint32_t* out_n_barcodes, BufPtr* out_barcode_spans, BufPtr* out_barcode_offsets,
-                                              BufPtr* out_ids) {
-    if (n_bytes >= 0xFFFFFFF0ull) return fail(GTGPU_ERR_UNSUPPORTED, "tokenize_fragments_text: at most 4 GiB of text per call");
+// tokenize_fragment_file from the file's text, any size: the barcodes come back as names.
+extern "C" int32_t gtgpu_tokenize_fragments_file(gtgpu_index* ix, const char* text, uint64_t n_bytes, uint32_t n_names,
+                                                 const char* names, const uint32_t* name_offsets, uint32_t unk_id,
+                                                 uint32_t* out_n_barcodes, gtgpu_buf** out_barcode_names,
+                                                 gtgpu_buf** out_barcode_name_offsets, gtgpu_buf** out_barcode_offsets,
+                                                 gtgpu_buf** out_ids) try {
+    if (!ix || !out_n_barcodes || !out_barcode_names || !out_barcode_name_offsets || !out_barcode_offsets || !out_ids ||
+        (n_bytes && !text) || (n_names && (!names || !name_offsets)))
+        return fail(GTGPU_ERR_INVALID, "tokenize_fragments_file: null argument");
     gtgpu_ctx* ctx = ix->ctx;
-    cudaStream_t st = ctx->stream;
-
-    uint32_t n = 0, n_barcodes = 0;
-    uint32_t *o_chr = nullptr, *o_start = nullptr, *o_end = nullptr, *d_bcid = nullptr, *d_spans = nullptr;
-    if (n_bytes) {
-        NameTable nt;
-        GT_TRY(upload_name_table(ctx, n_names, names, name_offsets, &nt));
-        const char* d_text = dev_text;
-        if (!dev_text) GT_TRY(ctx->scratch_get(SC_OUT_IDS2, n_bytes + 64, (void**)&d_text));
-        if (!dev_text) GT_CUDA(cudaMemcpyAsync((char*)d_text, host_text, n_bytes, cudaMemcpyHostToDevice, st));
-        FragParse fp;
-        GT_TRY(parse_fragments_locked(ctx, d_text, n_bytes, nt, FRAG_TOKENIZE, &fp));
-        if (fp.bad_line != 0xFFFFFFFFu)
-            return fail(GTGPU_ERR_INVALID, "tokenize_fragments_text: Invalid fragment file detected at line: " + std::to_string(fp.bad_line));
-        n = fp.n;
-        o_chr = fp.chr;
-        o_start = fp.start;
-        o_end = fp.end;
-        if (n) {
-            // ---- barcodes -> dense ids in first-appearance order -----------------------------------------------------------------
-            uint64_t cap = 1024;
-            while (cap < 2ull * n) cap <<= 1;
-            unsigned long long* d_keys;
-            uint32_t *d_first, *d_slot_of = fp.free0, *d_head = fp.free1, *d_rank = fp.free2;
-            uint32_t tail[2], flags[2];
-            GT_TRY(ctx->scratch_get(SC_BARCODE, (size_t)n * 4 + 8, (void**)&d_bcid));
-            GT_TRY(ctx->scratch_get(SC_MATRIX, cap * 12, (void**)&d_keys));
-            d_first = reinterpret_cast<uint32_t*>(d_keys + cap);
-            GT_CUDA(cudaMemsetAsync(d_keys, 0, cap * 8, st));
-            GT_CUDA(cudaMemsetAsync(d_first, 0xFF, cap * 4, st));
-            ingest_barcode_insert_kernel<<<igrid(ctx, n), 256, 0, st>>>(n, fp.h, (uint32_t)(cap - 1), d_keys, d_first, d_slot_of, 0u);
-            ingest_barcode_heads_kernel<<<igrid(ctx, n), 256, 0, st>>>(n, d_text, d_slot_of, d_first, fp.bo, fp.bl, d_head, fp.flags + 1);
-            ctx->launches += 2;
-            GT_TRY(exclusive_scan<uint32_t>(ctx, d_head, d_rank, n, fp.tmp));
-            GT_CUDA(cudaMemcpyAsync(&tail[0], d_rank + n - 1, 4, cudaMemcpyDeviceToHost, st));
-            GT_CUDA(cudaMemcpyAsync(&tail[1], d_head + n - 1, 4, cudaMemcpyDeviceToHost, st));
-            GT_CUDA(cudaMemcpyAsync(flags, fp.flags, 8, cudaMemcpyDeviceToHost, st));
-            GT_CUDA(cudaStreamSynchronize(st));
-            if (flags[1]) return fail(GTGPU_ERR_UNSUPPORTED, "tokenize_fragments_text: two barcodes share a 64-bit hash; use the array entry point");
-            n_barcodes = tail[0] + tail[1];
-            GT_TRY(ctx->scratch_get(SC_FILE_OFFS, (size_t)n_barcodes * 8 + 8, (void**)&d_spans));
-            ingest_barcode_ids_kernel<<<igrid(ctx, n), 256, 0, st>>>(n, d_slot_of, d_first, d_rank, fp.bo, fp.bl, d_bcid, d_spans);
-            ctx->launches++;
-            GT_CUDA(cudaGetLastError());
-        }
-    }
-    // ---- results -----------------------------------------------------------------------------------------------------------------
-    *out_n_barcodes = n_barcodes;
-    BufPtr spans, offs, ids;
-    const int32_t s = buf_from_device(ctx, d_spans, (uint64_t)n_barcodes * 2, 4, st, &spans);
-    if (s == GTGPU_ERR_CUDA) return fail(s, std::string("ingest: D2H: ") + gtgpu_last_error());
-    GT_TRY(s);
-    const cudaError_t e = cudaStreamSynchronize(st);
-    if (e != cudaSuccess) return fail(GTGPU_ERR_CUDA, std::string("ingest: D2H: ") + cudaGetErrorString(e));
-    GT_TRY(buf_new(ctx, (uint64_t)n_barcodes + 1, 8, &offs));
-    if (n) {
-        GT_TRY(tokenize_fragments_core(ix, n, o_chr, o_start, o_end, d_bcid, n_barcodes, unk_id, (uint64_t*)offs->block.ptr, &ids));
-    } else {
-        *(uint64_t*)offs->block.ptr = 0;
-        GT_TRY(buf_new(ctx, 0, 4, &ids));
-    }
-    *out_barcode_spans = std::move(spans);
-    *out_barcode_offsets = std::move(offs);
-    *out_ids = std::move(ids);
+    std::lock_guard<std::mutex> lk(ctx->mu);
+    GT_CUDA(cudaSetDevice(ctx->device));
+    BufPtr nm, no, offs, ids;
+    GT_TRY(tokenize_fragments_file_locked(ix, text, nullptr, n_bytes, n_names, names, name_offsets, unk_id, "tokenize_fragments_file",
+                                          out_n_barcodes, &nm, &no, nullptr, &offs, &ids));
+    *out_barcode_names = nm.release();
+    *out_barcode_name_offsets = no.release();
+    *out_barcode_offsets = offs.release();
+    *out_ids = ids.release();
     return GTGPU_OK;
-}
+} GT_CATCH

@@ -11,9 +11,6 @@
 //   barcodes: fused find with per-fragment offsets -> barcode of every hit -> two stable radix sorts (peak, then
 //             barcode) -> run-length encode -> CSR (barcode offsets, peaks, counts)
 #include <algorithm>
-#include <cstdlib>
-#include <cstring>
-#include <thread>
 
 #include "common.cuh"
 
@@ -365,128 +362,8 @@ extern "C" int32_t gtgpu_score_barcodes(gtgpu_index* ix, uint64_t n, const uint3
 } GT_CATCH
 
 // ---- region / barcode scoring from a fragment file's bytes -----------------------------------------------------------------
-// The text is parsed in windows (the parse kernels address a window with u32 positions): a window ends right after the first
-// '\n' at or past its nominal size, so it holds whole lines, and a window's local line index plus the lines of the windows
-// before it is the file-wide index the host parser reports.  Plain text is copied window by window (the copy of window k+1,
-// through pinned staging on the copy stream, overlaps the kernels of window k); gzip members are inflated whole into device
-// memory first and the windows run over that text.
+// Each file is parsed in windows (for_each_window, ingest.cu); gzip members are inflated whole into device memory first.
 namespace gtgpu {
-
-// GTGPU_INGEST_WINDOW=<bytes>, read per call: nominal window size (results never depend on it)
-static uint64_t ingest_window_bytes() {
-    uint64_t w = 2ull << 30;
-    if (const char* env = getenv("GTGPU_INGEST_WINDOW")) {
-        const uint64_t v = strtoull(env, nullptr, 10);
-        if (v) w = v;
-    }
-    return std::min<uint64_t>(w, 3ull << 30);
-}
-
-using WindowFn = std::function<int32_t(const char* d_window, uint64_t n_bytes, uint64_t first_line, uint32_t* n_lines)>;
-
-struct StagingScope {  // pinned staging blocks and their events, returned to the ctx when the call ends
-    gtgpu_ctx* ctx;
-    PinnedBlock pin[2];
-    cudaEvent_t ev[2] = {nullptr, nullptr};
-    bool used[2] = {false, false};
-    explicit StagingScope(gtgpu_ctx* c) : ctx(c) {}
-    ~StagingScope() {
-        cudaStreamSynchronize(ctx->copy_in);
-        for (int b = 0; b < 2; ++b) {
-            if (ev[b]) cudaEventDestroy(ev[b]);
-            ctx->pinned_put(pin[b]);
-        }
-    }
-};
-
-// Exactly one of host_text / dev_text is given.  The caller holds ctx->mu.
-static int32_t for_each_window(gtgpu_ctx* ctx, const char* host_text, const char* dev_text, uint64_t n_bytes, const std::string& who,
-                               const WindowFn& fn) {
-    cudaStream_t st = ctx->stream;
-    const uint64_t W = ingest_window_bytes();
-    std::vector<uint64_t> cut{0};  // window w = [cut[w], cut[w + 1])
-    while (cut.back() < n_bytes) {
-        const uint64_t a = cut.back();
-        uint64_t b = n_bytes;
-        if (n_bytes - a > W) {
-            const uint64_t p = a + W - 1;
-            if (host_text) {
-                const void* q = memchr(host_text + p, '\n', n_bytes - p);
-                if (q) b = (uint64_t)((const char*)q - host_text) + 1;
-            } else {
-                char piece[4096];
-                for (uint64_t q = p; q < n_bytes && b == n_bytes; q += sizeof piece) {
-                    const uint64_t len = std::min<uint64_t>(sizeof piece, n_bytes - q);
-                    GT_CUDA(cudaMemcpyAsync(piece, dev_text + q, len, cudaMemcpyDeviceToHost, st));
-                    GT_CUDA(cudaStreamSynchronize(st));
-                    const void* nl = memchr(piece, '\n', len);
-                    if (nl) b = q + (uint64_t)((const char*)nl - piece) + 1;
-                }
-            }
-        }
-        if (b - a >= 0xFFFFFFF0ull) return fail(GTGPU_ERR_UNSUPPORTED, who + ": a line of 4 GiB or more");
-        cut.push_back(b);
-    }
-    const size_t n_win = cut.size() - 1;
-    uint64_t max_win = 0;
-    for (size_t w = 0; w < n_win; ++w) max_win = std::max(max_win, cut[w + 1] - cut[w]);
-    uint64_t first_line = 0;
-    uint32_t n_lines = 0;
-    if (dev_text) {
-        char* d_copy = nullptr;  // windows that do not start 16-byte aligned are moved to aligned scratch (the newline scan loads 16 B)
-        for (size_t w = 0; w < n_win; ++w) {
-            const char* d = dev_text + cut[w];
-            if (reinterpret_cast<uintptr_t>(d) & 15) {
-                if (!d_copy) GT_TRY(ctx->scratch_get(SC_WIN_A, max_win + 64, (void**)&d_copy));
-                GT_CUDA(cudaMemcpyAsync(d_copy, d, cut[w + 1] - cut[w], cudaMemcpyDeviceToDevice, st));
-                d = d_copy;
-            }
-            GT_TRY(fn(d, cut[w + 1] - cut[w], first_line, &n_lines));
-            first_line += n_lines;
-        }
-        return GTGPU_OK;
-    }
-    char* dbuf[2] = {nullptr, nullptr};
-    GT_TRY(ctx->scratch_get(SC_WIN_A, max_win + 64, (void**)&dbuf[0]));
-    if (n_win > 1) GT_TRY(ctx->scratch_get(SC_WIN_B, max_win + 64, (void**)&dbuf[1]));
-    StagingScope sg(ctx);
-    const uint64_t piece = std::min<uint64_t>(max_win, 64ull << 20);
-    for (int b = 0; b < 2; ++b) {
-        GT_TRY(ctx->pinned_get(piece, &sg.pin[b]));
-        GT_CUDA(cudaEventCreateWithFlags(&sg.ev[b], cudaEventDisableTiming));
-    }
-    // window w -> dbuf[w % 2] through the two pinned pieces; runs on a helper thread while the kernels of window w - 1 run
-    std::string stage_err;
-    auto stage = [&](size_t w) -> int32_t {
-        if (cudaSetDevice(ctx->device) != cudaSuccess) return GTGPU_ERR_CUDA;
-        cudaError_t e = cudaSuccess;
-        uint64_t j = 0;
-        for (uint64_t off = cut[w]; off < cut[w + 1] && e == cudaSuccess; off += piece, ++j) {
-            const int b = (int)(j & 1);
-            const uint64_t len = std::min(piece, cut[w + 1] - off);
-            if (sg.used[b]) e = cudaEventSynchronize(sg.ev[b]);
-            if (e != cudaSuccess) break;
-            memcpy(sg.pin[b].ptr, host_text + off, len);
-            e = cudaMemcpyAsync(dbuf[w & 1] + (off - cut[w]), sg.pin[b].ptr, len, cudaMemcpyHostToDevice, ctx->copy_in);
-            if (e == cudaSuccess) e = cudaEventRecord(sg.ev[b], ctx->copy_in);
-            sg.used[b] = true;
-        }
-        if (e == cudaSuccess) e = cudaStreamSynchronize(ctx->copy_in);
-        if (e != cudaSuccess) stage_err = std::string("H2D of the text: ") + cudaGetErrorString(e);
-        return e == cudaSuccess ? GTGPU_OK : GTGPU_ERR_CUDA;
-    };
-    int32_t s_next = stage(0);
-    for (size_t w = 0; w < n_win && s_next == GTGPU_OK; ++w) {
-        std::thread helper;
-        if (w + 1 < n_win) helper = std::thread([&, w] { s_next = stage(w + 1); });
-        const int32_t s = fn(dbuf[w & 1], cut[w + 1] - cut[w], first_line, &n_lines);
-        if (helper.joinable()) helper.join();
-        if (s != GTGPU_OK) return s;
-        first_line += n_lines;
-    }
-    if (s_next != GTGPU_OK) return fail(s_next, who + ": " + stage_err);
-    return GTGPU_OK;
-}
 
 static int32_t parse_error(const std::string& who, uint64_t line) {
     return fail(GTGPU_ERR_INVALID, who + ": Failed to parse fragment at line " + std::to_string(line));
@@ -512,7 +389,7 @@ static int32_t score_matrix_text_locked(gtgpu_index* ix, const char* host_text, 
         GT_TRY(upload_name_table(ctx, n_names, names, name_offsets, &nt));
         GT_TRY(ctx->scratch_get(SC_FILE_OFFS, 16, (void**)&d_fo));
         GT_TRY(for_each_window(ctx, host_text, dev_text, n_bytes, who,
-                               [&](const char* d, uint64_t nb, uint64_t line0, uint32_t* n_lines) -> int32_t {
+                               [&](const char* d, uint64_t nb, uint64_t, uint64_t line0, uint32_t* n_lines) -> int32_t {
             FragParse fp;
             GT_TRY(parse_fragments_locked(ctx, d, nb, nt, FRAG_SCORE_MATRIX, &fp));
             *n_lines = fp.n_lines;
@@ -537,18 +414,18 @@ static int32_t score_barcodes_text_locked(gtgpu_index* ix, const char* host_text
                                           gtgpu_buf** out_names, gtgpu_buf** out_name_offsets, gtgpu_buf** out_barcode_offsets,
                                           gtgpu_buf** out_peaks, gtgpu_buf** out_counts, const std::string& who) {
     gtgpu_ctx* ctx = ix->ctx;
-    FragBarcodeTable tab;
+    FragBarcodeTable tab(false, false, who, "gtgpu_score_barcodes");
     if (n_bytes) {
         NameTable nt;
         GT_TRY(upload_name_table(ctx, n_names, names, name_offsets, &nt));
         GT_TRY(for_each_window(ctx, host_text, dev_text, n_bytes, who,
-                               [&](const char* d, uint64_t nb, uint64_t line0, uint32_t* n_lines) -> int32_t {
+                               [&](const char* d, uint64_t nb, uint64_t byte0, uint64_t line0, uint32_t* n_lines) -> int32_t {
             FragParse fp;
             GT_TRY(parse_fragments_locked(ctx, d, nb, nt, FRAG_SCORE_BARCODES, &fp));
             *n_lines = fp.n_lines;
             if (fp.bad_line != 0xFFFFFFFFu) return parse_error(who, line0 + fp.bad_line);
             if (tab.n + fp.n > 0xFFFFFFFFull) return too_many(who);
-            return tab.add_window(ctx, d, fp, n_names);
+            return tab.add_window(ctx, d, byte0, fp, n_names);
         }));
     }
     uint32_t n_kept = 0;
@@ -562,16 +439,6 @@ static int32_t score_barcodes_text_locked(gtgpu_index* ix, const char* host_text
     *out_name_offsets = no.release();
     *out_barcode_offsets = offs.release();
     return GTGPU_OK;
-}
-
-// gzip members -> device text (SC_GZ_OUT); a text that does not fit in device memory is reported as such
-static int32_t inflate_for_scoring(gtgpu_ctx* ctx, uint64_t n_members, const uint8_t* gz, const uint64_t* member_offsets,
-                                   const std::string& who, uint8_t** d_text, uint64_t* n_text) {
-    const int32_t s = gunzip_locked(ctx, n_members, gz, member_offsets, nullptr, d_text, n_text);
-    if (s == GTGPU_ERR_NOMEM)
-        return fail(s, who + ": the inflated text does not fit in device memory (gzip input is inflated whole before it is parsed): " +
-                           gtgpu_last_error());
-    return s;
 }
 
 }  // namespace gtgpu
@@ -598,7 +465,7 @@ extern "C" int32_t gtgpu_score_matrix_gz(gtgpu_index* ix, uint64_t n_members, co
     GT_CUDA(cudaSetDevice(ctx->device));
     uint8_t* d_text = nullptr;
     uint64_t n_text = 0;
-    GT_TRY(inflate_for_scoring(ctx, n_members, gz, member_offsets, "score_matrix_gz", &d_text, &n_text));
+    GT_TRY(inflate_whole_locked(ctx, n_members, gz, member_offsets, "score_matrix_gz", &d_text, &n_text));
     return score_matrix_text_locked(ix, nullptr, (const char*)d_text, n_text, n_names, names, name_offsets, mode, n_cols, out_row,
                                     "score_matrix_gz");
 } GT_CATCH
@@ -630,7 +497,7 @@ extern "C" int32_t gtgpu_score_barcodes_gz(gtgpu_index* ix, uint64_t n_members, 
     GT_CUDA(cudaSetDevice(ctx->device));
     uint8_t* d_text = nullptr;
     uint64_t n_text = 0;
-    GT_TRY(inflate_for_scoring(ctx, n_members, gz, member_offsets, "score_barcodes_gz", &d_text, &n_text));
+    GT_TRY(inflate_whole_locked(ctx, n_members, gz, member_offsets, "score_barcodes_gz", &d_text, &n_text));
     return score_barcodes_text_locked(ix, nullptr, (const char*)d_text, n_text, n_names, names, name_offsets, out_n_barcodes,
                                       out_barcode_names, out_barcode_name_offsets, out_barcode_offsets, out_peaks, out_counts,
                                       "score_barcodes_gz");

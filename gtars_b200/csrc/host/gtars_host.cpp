@@ -715,28 +715,30 @@ std::vector<std::pair<std::string, std::vector<uint32_t>>> Tokenizer::tokenize_f
 std::vector<std::pair<std::string, std::vector<uint32_t>>> Tokenizer::tokenize_fragment_file_device(const std::string& path) const {
     NameBlob nb(cmap_);
     uint32_t n_barcodes = 0;
-    PinnedResult spans, offs, ids, dev_text;
-    std::string raw, host_text;
-    std::vector<uint64_t> members;
-    const char* text = nullptr;
-    if (gz_members_for_device(path, raw, members)) {  // bgzip'ed fragment file: inflated on the device, the text comes back once
-        check(gtgpu_tokenize_fragments_gz(index_, members.size() - 1, (const uint8_t*)raw.data(), members.data(), (uint32_t)cmap_.size(),
-                                          nb.blob.data(), nb.offsets.data(), unk_id_, &n_barcodes, &spans.buf, &offs.buf, &ids.buf,
-                                          &dev_text.buf),
-              "gtgpu_tokenize_fragments_gz");
-        text = (const char*)gtgpu_buf_data(dev_text.buf);
-    } else {
-        host_text = read_file_bytes(path);
-        check(gtgpu_tokenize_fragments_text(index_, host_text.data(), host_text.size(), (uint32_t)cmap_.size(), nb.blob.data(),
-                                            nb.offsets.data(), unk_id_, &n_barcodes, &spans.buf, &offs.buf, &ids.buf),
-              "gtgpu_tokenize_fragments_text");
-        text = host_text.data();
+    PinnedResult names, name_offsets, offs, ids;
+    {
+        std::string raw;
+        std::vector<uint64_t> members;
+        if (gz_members_for_device(path, raw, members)) {  // bgzip'ed fragment file: inflated and parsed on the device
+            check(gtgpu_tokenize_fragments_file_gz(index_, members.size() - 1, (const uint8_t*)raw.data(), members.data(),
+                                                   (uint32_t)cmap_.size(), nb.blob.data(), nb.offsets.data(), unk_id_, &n_barcodes,
+                                                   &names.buf, &name_offsets.buf, &offs.buf, &ids.buf),
+                  "gtgpu_tokenize_fragments_file_gz");
+        } else {
+            const std::string text = read_file_bytes(path);
+            check(gtgpu_tokenize_fragments_file(index_, text.data(), text.size(), (uint32_t)cmap_.size(), nb.blob.data(),
+                                                nb.offsets.data(), unk_id_, &n_barcodes, &names.buf, &name_offsets.buf, &offs.buf,
+                                                &ids.buf),
+                  "gtgpu_tokenize_fragments_file");
+        }
     }
+    const char* blob = (const char*)gtgpu_buf_data(names.buf);
+    const uint64_t* noff = (const uint64_t*)gtgpu_buf_data(name_offsets.buf);
     const uint64_t* off = (const uint64_t*)gtgpu_buf_data(offs.buf);
     std::vector<std::pair<std::string, std::vector<uint32_t>>> out;
     out.reserve(n_barcodes);
     for (uint32_t b = 0; b < n_barcodes; ++b)
-        out.emplace_back(std::string(text + spans.data()[2 * b], spans.data()[2 * b + 1]),
+        out.emplace_back(std::string(blob + noff[b], noff[b + 1] - noff[b]),
                          std::vector<uint32_t>(ids.data() + off[b], ids.data() + off[b + 1]));
     return out;
 }

@@ -212,8 +212,8 @@ class Tokenizer {
     std::vector<std::string> decode(const std::vector<uint32_t>& ids) const;      // tokenizer.rs:173-181
     // utils/fragments.rs:61-82: barcode -> token ids, every fragment one tokenize() call (per-fragment [unk]).
     std::vector<std::pair<std::string, std::vector<uint32_t>>> tokenize_fragment_file(const std::string& path) const;
-    // The same with the file's text parsed, barcodes numbered and fragments tokenized on the device
-    // (gtgpu_tokenize_fragments_text); barcodes come back in first-appearance order.
+    // The same with the file's text (any size; a bgzip'ed file is inflated on the device) parsed, barcodes numbered and
+    // fragments tokenized on the device (gtgpu_tokenize_fragments_file / _gz); barcodes come back in first-appearance order.
     std::vector<std::pair<std::string, std::vector<uint32_t>>> tokenize_fragment_file_device(const std::string& path) const;
     // utils/fragments.rs:87-112: barcode -> (token id -> count).
     std::vector<std::pair<std::string, std::map<uint32_t, uint32_t>>> count_fragments_by_barcode(const std::string& path) const;

@@ -232,7 +232,8 @@ int32_t gtgpu_tokenize_bed(gtgpu_index* index, const char* text, uint64_t n_byte
  * (64-bit FNV-1a + byte comparison against the first appearance; a true hash collision is reported as
  * GTGPU_ERR_UNSUPPORTED).  Outputs: *out_n_barcodes; *out_barcode_spans = (byte offset, length) of each barcode's first
  * occurrence in `text` (u32 pairs, so the caller recovers the strings); *out_barcode_offsets = n_barcodes + 1 u64
- * offsets into *out_ids (gtgpu_buf_len counts 8-byte elements); ids as gtgpu_tokenize_fragments returns them. */
+ * offsets into *out_ids (gtgpu_buf_len counts 8-byte elements); ids as gtgpu_tokenize_fragments returns them.  n_bytes < 4 GiB
+ * (GTGPU_ERR_UNSUPPORTED beyond); gtgpu_tokenize_fragments_file takes any size and returns the names themselves. */
 int32_t gtgpu_tokenize_fragments_text(gtgpu_index* index, const char* text, uint64_t n_bytes, uint32_t n_names,
                                       const char* names, const uint32_t* name_offsets, uint32_t unk_id,
                                       uint32_t* out_n_barcodes, gtgpu_buf** out_barcode_spans,
@@ -265,6 +266,25 @@ int32_t gtgpu_tokenize_fragments_gz(gtgpu_index* index, uint64_t n_members, cons
                                     uint32_t n_names, const char* names, const uint32_t* name_offsets, uint32_t unk_id,
                                     uint32_t* out_n_barcodes, gtgpu_buf** out_barcode_spans, gtgpu_buf** out_barcode_offsets,
                                     gtgpu_buf** out_ids, gtgpu_buf** out_text);
+
+/* tokenize_fragment_file from ONE fragment file's bytes of any size, parsed on the device: the (decompressed) text, or its gzip
+ * members (n_members, gz, member_offsets as in gtgpu_gunzip; inflated whole into device memory, GTGPU_ERR_NOMEM when that text
+ * does not fit).  Line rules, chromosome names, malformed-line errors ("Invalid fragment file detected at line: i", 0-based,
+ * '#' lines count, no output) and results are those of gtgpu_tokenize_fragments_text: every barcode is kept, including one
+ * whose fragments all lie on unknown chromosomes.  The text is parsed in windows of about GTGPU_INGEST_WINDOW bytes (default
+ * 2 GiB), as the scoring entry points do; at most 2^32 - 1 fragments per file and no more ids than gtgpu_tokenize_fragments
+ * takes (GTGPU_ERR_UNSUPPORTED beyond).  Outputs: *out_n_barcodes; *out_barcode_names = the barcodes' bytes back to back in
+ * first-appearance order (u8 elements); *out_barcode_name_offsets = n_barcodes + 1 u64 offsets into those bytes;
+ * *out_barcode_offsets = n_barcodes + 1 u64 offsets into *out_ids (u32), as gtgpu_tokenize_fragments returns them.  On a
+ * multi-device ctx these run on the first device.  gtgpu_tokenize_fragments_text / _gz run on the same windowed parse. */
+int32_t gtgpu_tokenize_fragments_file(gtgpu_index* index, const char* text, uint64_t n_bytes, uint32_t n_names, const char* names,
+                                      const uint32_t* name_offsets, uint32_t unk_id, uint32_t* out_n_barcodes,
+                                      gtgpu_buf** out_barcode_names, gtgpu_buf** out_barcode_name_offsets,
+                                      gtgpu_buf** out_barcode_offsets, gtgpu_buf** out_ids);
+int32_t gtgpu_tokenize_fragments_file_gz(gtgpu_index* index, uint64_t n_members, const uint8_t* gz, const uint64_t* member_offsets,
+                                         uint32_t n_names, const char* names, const uint32_t* name_offsets, uint32_t unk_id,
+                                         uint32_t* out_n_barcodes, gtgpu_buf** out_barcode_names, gtgpu_buf** out_barcode_name_offsets,
+                                         gtgpu_buf** out_barcode_offsets, gtgpu_buf** out_ids);
 
 /* ---- gtars-scoring: fragments x consensus peaks ------------------------------------------------------------------------
  * gtgpu_score_matrix replaces region_scoring_from_fragments (gtars-scoring/src/fragment_scoring.rs:19-121) over
