@@ -124,6 +124,15 @@ extern "C" {
                                    out_counts: *mut *mut gtgpu_buf) -> i32;
     pub fn gtgpu_igd_build(ctx: *mut gtgpu_ctx, n_files: u64, file_offsets: *const u64, n_chroms: u32, chr: *const u32,
                            start: *const u32, end: *const u32, out_igd: *mut *mut gtgpu_igd) -> i32;
+    /// An IGD from its BED files' text (file f = text[file_offsets[f], file_offsets[f + 1]), any size), parsed on the device;
+    /// the chromosome names come back in id order (bytes + n_chroms + 1 u64 offsets).
+    pub fn gtgpu_igd_build_bed(ctx: *mut gtgpu_ctx, n_files: u64, text: *const c_char, file_offsets: *const u64, out_n_chroms: *mut u32,
+                               out_chrom_names: *mut *mut gtgpu_buf, out_chrom_name_offsets: *mut *mut gtgpu_buf,
+                               out_igd: *mut *mut gtgpu_igd) -> i32;
+    /// The same from gzip members: file f = members [file_members[f], file_members[f + 1]) of gz / member_offsets.
+    pub fn gtgpu_igd_build_bed_gz(ctx: *mut gtgpu_ctx, n_files: u64, file_members: *const u64, n_members: u64, gz: *const u8,
+                                  member_offsets: *const u64, out_n_chroms: *mut u32, out_chrom_names: *mut *mut gtgpu_buf,
+                                  out_chrom_name_offsets: *mut *mut gtgpu_buf, out_igd: *mut *mut gtgpu_igd) -> i32;
     pub fn gtgpu_igd_free(igd: *mut gtgpu_igd) -> i32;
     pub fn gtgpu_igd_info(igd: *const gtgpu_igd, info: *mut u64) -> i32;
     pub fn gtgpu_igd_count_set_overlaps(igd: *mut gtgpu_igd, n_sets: u64, set_offsets: *const u64, chr: *const u32,

@@ -61,6 +61,7 @@ def lib():
             "gth_igd_single": (vp, [vp, vp]), "gth_igd_find_pairs": (vp, [vp, vp, i32]),
             "gth_igd_count_per_query": (vp, [vp, vp, i32]),
             "gth_igd_save_sets": (C.c_int, [u64, vp, vp, cp]), "gth_igd_from_file": (vp, [vp, cp]),
+            "gth_igd_from_bed_files": (vp, [vp, u64, vp]), "gth_igd_info": (C.c_int, [vp, vp]),
             "gth_igd_new": (vp, [vp, u64, vp]), "gth_igd_free": (None, [vp]), "gth_igd_num_files": (u64, [vp]),
             "gth_igd_count": (C.c_int, [vp, u64, vp, i32, C.c_int, vp]),
             "gth_lola_contingency": (C.c_int, [vp, u64, vp, vp, i32, vp]),
@@ -480,6 +481,25 @@ class Igd:
         if not obj._h:
             _fail()
         return obj
+
+    @classmethod
+    def from_bed_files(cls, paths):
+        """Igd([RegionSet(p) for p in paths]) with the files' text parsed on the device, their regions never on the host
+        (gtgpu_igd_build_bed; when every path ends in .gz the gzip bytes are inflated on the device too)."""
+        paths = [os.fsencode(p) for p in paths]
+        obj = cls.__new__(cls)
+        obj._sets = []
+        obj._h = lib().gth_igd_from_bed_files(device(), len(paths), (C.c_char_p * max(len(paths), 1))(*paths))
+        if not obj._h:
+            _fail()
+        return obj
+
+    def info(self) -> dict:
+        """gtgpu_igd_info of a database Igd: files, records kept, device bytes, LUT shift."""
+        a = np.zeros(4, dtype=np.uint64)
+        if lib().gth_igd_info(self._h, a.ctypes.data):
+            _fail()
+        return dict(n_files=int(a[0]), n_records=int(a[1]), device_bytes=int(a[2]), lut_shift=int(a[3]))
 
     @classmethod
     def from_single_region_set(cls, subject):

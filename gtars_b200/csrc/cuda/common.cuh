@@ -338,6 +338,15 @@ struct NameTable {
     const uint32_t* hash_id;      // name id of the k-th sorted hash
     uint32_t n_names;
 };
+// What the BED line kernel needs to parse a text of several files back to back (ingest_parse_lines_kernel<true>).
+struct BedFilesView {
+    const unsigned long long* file_offsets = nullptr;  // n_files + 1 byte offsets of the files in the whole text
+    uint64_t n_files = 0;
+    uint64_t byte0 = 0, line0 = 0;                     // the window's first byte and first line in the whole text
+    unsigned long long* first_line = nullptr;          // [f] = text-wide index of file f's first line
+    unsigned long long* name_hash = nullptr;           // per line: FNV-1a of the chromosome name (never 0), its window
+    uint32_t *name_off = nullptr, *name_len = nullptr;  // offset and length
+};
 // the caller's chromosome names -> scratch SC_SET_ID
 int32_t upload_name_table(gtgpu_ctx* ctx, uint32_t n_names, const char* names, const uint32_t* name_offsets, NameTable* out);
 // What the fragment parse checks and carries: tokenize_fragment_file needs fields 1 and 2 as u32 and the barcode;
@@ -399,7 +408,7 @@ int32_t gunzip_locked(gtgpu_ctx* ctx, uint64_t n_members, const uint8_t* gz, con
                       uint64_t* out_member_offsets, uint8_t** d_text, uint64_t* n_text);
 // gunzip_locked for a text parsed in windows afterwards: a text that does not fit in device memory is reported as such
 int32_t inflate_whole_locked(gtgpu_ctx* ctx, uint64_t n_members, const uint8_t* gz, const uint64_t* member_offsets, const std::string& who,
-                             uint8_t** d_text, uint64_t* n_text);
+                             uint8_t** d_text, uint64_t* n_text, uint64_t* out_member_offsets = nullptr);
 // The text is host_text (copied to the device here) or dev_text (already there, e.g. inflated): exactly one is non-null.
 int32_t tokenize_bed_locked(gtgpu_index* ix, const char* host_text, const char* dev_text, uint64_t n_bytes, uint32_t n_names,
                             const char* names, const uint32_t* name_offsets, uint32_t unk_id, gtgpu_buf** out_ids);
@@ -409,6 +418,20 @@ int32_t tokenize_fragments_file_locked(gtgpu_index* ix, const char* host_text, c
                                        const char* names, const uint32_t* name_offsets, uint32_t unk_id, const std::string& who,
                                        uint32_t* out_n_barcodes, BufPtr* out_names, BufPtr* out_name_offsets, BufPtr* out_spans,
                                        BufPtr* out_barcode_offsets, BufPtr* out_ids);
+
+// The region lines of n_files BED files back to back (file f = text[file_offsets[f], file_offsets[f + 1]), any total size),
+// parsed on the device in windows: line rules of gtgpu_parse_bed per file, chromosome names discovered in first-appearance order.
+// On success chr / start / end / file hold the n records in file order (chr = dense name id), file_offsets the files' record
+// offsets (n_files + 1), names / name_offsets the chromosome names in id order.  The caller holds ctx->mu.
+struct BedFilesRecords {
+    DevMem chr, start, end, file;
+    uint64_t n = 0;
+    std::vector<uint64_t> file_offsets;
+    std::string names;
+    std::vector<uint64_t> name_offsets;
+};
+int32_t parse_bed_files_locked(gtgpu_ctx* ctx, const char* host_text, const char* dev_text, uint64_t n_files, const uint64_t* file_offsets,
+                               const std::string& who, BedFilesRecords* out);
 
 // groups (api.cu, comm.cu, igd.cu)
 int32_t for_each_device(size_t n_devices, const std::function<int32_t(size_t)>& fn);

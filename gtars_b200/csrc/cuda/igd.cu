@@ -305,6 +305,8 @@ using namespace gtgpu;
 // builds its own record pool over sets [r * C, min((r + 1) * C, n_files)), C = ceil(n_files / devices), all in parallel.
 static int32_t igd_build_one(gtgpu_ctx* ctx, uint64_t n_files, const uint64_t* file_offsets, uint32_t n_chroms, const uint32_t* chr,
                              const uint32_t* start, const uint32_t* end, gtgpu_igd** out_igd);
+static int32_t igd_build_dev(gtgpu_ctx* ctx, uint64_t n_files, uint32_t n_chroms, uint64_t total, const uint32_t* t_chr,
+                             const uint32_t* t_start, const uint32_t* t_end, const uint32_t* t_file, gtgpu_igd** out_igd);
 
 static int32_t igd_build_group(gtgpu_ctx* ctx, uint64_t n_files, const uint64_t* file_offsets, uint32_t n_chroms, const uint32_t* chr,
                                const uint32_t* start, const uint32_t* end, gtgpu_igd** out_igd) {
@@ -353,11 +355,115 @@ extern "C" int32_t gtgpu_igd_build(gtgpu_ctx* ctx, uint64_t n_files, const uint6
     return igd_build_one(ctx, n_files, file_offsets, n_chroms, chr, start, end, out_igd);
 } GT_CATCH
 
+// ---- a database from its BED files' text, parsed on the device --------------------------------------------------------------
+// The records and the chromosome names come from parse_bed_files_locked on ctx (the first device of a group).  One device: the
+// build reads the parsed records where they are.  A group: shard r's files are a contiguous record range, copied to its
+// device with cudaMemcpyAsync by the builder of gtgpu_igd_build (igd_records_to_device).
+static int32_t igd_build_parsed(gtgpu_ctx* ctx, uint64_t n_files, BedFilesRecords& r, uint32_t* out_n_chroms, gtgpu_buf** out_names,
+                                gtgpu_buf** out_name_offsets, gtgpu_igd** out_igd) {
+    const uint32_t n_chroms = (uint32_t)(r.name_offsets.size() - 1);
+    BufPtr names, offsets;
+    GT_TRY(buf_new(ctx, r.names.size(), 1, &names));
+    GT_TRY(buf_new(ctx, n_chroms + 1, 8, &offsets));
+    if (!r.names.empty()) memcpy(names->block.ptr, r.names.data(), r.names.size());
+    memcpy(offsets->block.ptr, r.name_offsets.data(), (n_chroms + 1) * 8);
+    gtgpu_igd* g = nullptr;
+    if (ctx->peers.size() > 1) {
+        GT_TRY(igd_build_group(ctx, n_files, r.file_offsets.data(), n_chroms, r.chr.u32(), r.start.u32(), r.end.u32(), &g));
+        GT_CUDA(cudaSetDevice(ctx->device));  // the parsed records are freed on their device
+    } else {
+        std::lock_guard<std::mutex> lk(ctx->mu);
+        GT_CUDA(cudaSetDevice(ctx->device));
+        GT_TRY(igd_build_dev(ctx, n_files, n_chroms, r.n, r.chr.u32(), r.start.u32(), r.end.u32(), r.file.u32(), &g));
+    }
+    *out_n_chroms = n_chroms;
+    *out_names = names.release();
+    *out_name_offsets = offsets.release();
+    *out_igd = g;
+    return GTGPU_OK;
+}
+
+extern "C" int32_t gtgpu_igd_build_bed(gtgpu_ctx* ctx, uint64_t n_files, const char* text, const uint64_t* file_offsets,
+                                       uint32_t* out_n_chroms, gtgpu_buf** out_chrom_names, gtgpu_buf** out_chrom_name_offsets,
+                                       gtgpu_igd** out_igd) try {
+    if (!ctx || !file_offsets || !out_n_chroms || !out_chrom_names || !out_chrom_name_offsets || !out_igd)
+        return fail(GTGPU_ERR_INVALID, "igd_build_bed: null argument");
+    if (file_offsets[0] != 0) return fail(GTGPU_ERR_INVALID, "igd_build_bed: file_offsets[0] must be 0");
+    for (uint64_t f = 0; f < n_files; ++f)
+        if (file_offsets[f] > file_offsets[f + 1]) return fail(GTGPU_ERR_INVALID, "igd_build_bed: file_offsets not monotone");
+    if (file_offsets[n_files] && !text) return fail(GTGPU_ERR_INVALID, "igd_build_bed: null text");
+    if (n_files >= 0xFFFFFFFFull) return fail(GTGPU_ERR_UNSUPPORTED, "igd_build_bed: too many files");
+    BedFilesRecords r;
+    {
+        std::lock_guard<std::mutex> lk(ctx->mu);
+        GT_CUDA(cudaSetDevice(ctx->device));
+        GT_TRY(parse_bed_files_locked(ctx, text, nullptr, n_files, file_offsets, "igd_build_bed", &r));
+    }
+    return igd_build_parsed(ctx, n_files, r, out_n_chroms, out_chrom_names, out_chrom_name_offsets, out_igd);
+} GT_CATCH
+
+extern "C" int32_t gtgpu_igd_build_bed_gz(gtgpu_ctx* ctx, uint64_t n_files, const uint64_t* file_members, uint64_t n_members,
+                                          const uint8_t* gz, const uint64_t* member_offsets, uint32_t* out_n_chroms,
+                                          gtgpu_buf** out_chrom_names, gtgpu_buf** out_chrom_name_offsets, gtgpu_igd** out_igd) try {
+    if (!ctx || !file_members || !out_n_chroms || !out_chrom_names || !out_chrom_name_offsets || !out_igd)
+        return fail(GTGPU_ERR_INVALID, "igd_build_bed_gz: null argument");
+    GT_TRY(check_members(n_members, gz, member_offsets, "igd_build_bed_gz"));
+    if (file_members[0] != 0 || file_members[n_files] != n_members)
+        return fail(GTGPU_ERR_INVALID, "igd_build_bed_gz: file_members must run from 0 to n_members");
+    for (uint64_t f = 0; f < n_files; ++f)
+        if (file_members[f] > file_members[f + 1]) return fail(GTGPU_ERR_INVALID, "igd_build_bed_gz: file_members not monotone");
+    if (n_files >= 0xFFFFFFFFull) return fail(GTGPU_ERR_UNSUPPORTED, "igd_build_bed_gz: too many files");
+    BedFilesRecords r;
+    {
+        std::lock_guard<std::mutex> lk(ctx->mu);
+        GT_CUDA(cudaSetDevice(ctx->device));
+        uint8_t* d_text = nullptr;
+        uint64_t n_text = 0;
+        std::vector<uint64_t> text_offsets(n_members + 1), fo(n_files + 1);
+        GT_TRY(inflate_whole_locked(ctx, n_members, gz, member_offsets, "igd_build_bed_gz", &d_text, &n_text, text_offsets.data()));
+        for (uint64_t f = 0; f <= n_files; ++f) fo[f] = text_offsets[file_members[f]];
+        GT_TRY(parse_bed_files_locked(ctx, nullptr, (const char*)d_text, n_files, fo.data(), "igd_build_bed_gz", &r));
+    }
+    return igd_build_parsed(ctx, n_files, r, out_n_chroms, out_chrom_names, out_chrom_name_offsets, out_igd);
+} GT_CATCH
+
+// Records to the device: chr / start / end (host or device memory, any device: cudaMemcpyDefault) into temporaries of tp, and
+// every record's file index from file_offsets.
+static int32_t igd_records_to_device(gtgpu_ctx* ctx, TempPool& tp, uint64_t n_files, const uint64_t* file_offsets, const uint32_t* chr,
+                                     const uint32_t* start, const uint32_t* end, uint32_t** t_chr, uint32_t** t_start, uint32_t** t_end,
+                                     uint32_t** t_file) {
+    const uint64_t total = file_offsets[n_files];
+    cudaStream_t st = ctx->stream;
+    uint64_t* t_fo;
+    GT_TRY(tp.get(total, t_chr));
+    GT_TRY(tp.get(total, t_start));
+    GT_TRY(tp.get(total, t_end));
+    GT_TRY(tp.get(total, t_file));
+    GT_TRY(tp.get(n_files + 1, &t_fo));
+    if (total) {
+        GT_CUDA(cudaMemcpyAsync(*t_chr, chr, total * 4, cudaMemcpyDefault, st));
+        GT_CUDA(cudaMemcpyAsync(*t_start, start, total * 4, cudaMemcpyDefault, st));
+        GT_CUDA(cudaMemcpyAsync(*t_end, end, total * 4, cudaMemcpyDefault, st));
+    }
+    GT_CUDA(cudaMemcpyAsync(t_fo, file_offsets, (n_files + 1) * 8, cudaMemcpyHostToDevice, st));
+    GT_CUDA(cudaStreamSynchronize(st));  // the caller's arrays may be pageable
+    if (total) GT_TRY(launch_fill_set_ids(ctx, n_files, t_fo, *t_file));
+    return GTGPU_OK;
+}
+
 static int32_t igd_build_one(gtgpu_ctx* ctx, uint64_t n_files, const uint64_t* file_offsets, uint32_t n_chroms, const uint32_t* chr,
                              const uint32_t* start, const uint32_t* end, gtgpu_igd** out_igd) {
-    const uint64_t total = file_offsets[n_files];
     std::lock_guard<std::mutex> lk(ctx->mu);
     GT_CUDA(cudaSetDevice(ctx->device));
+    TempPool tp;
+    uint32_t *t_chr, *t_start, *t_end, *t_file;
+    GT_TRY(igd_records_to_device(ctx, tp, n_files, file_offsets, chr, start, end, &t_chr, &t_start, &t_end, &t_file));
+    return igd_build_dev(ctx, n_files, n_chroms, file_offsets[n_files], t_chr, t_start, t_end, t_file, out_igd);
+}
+
+// The build from device-resident records of this ctx's device (record i belongs to file t_file[i]).  The caller holds ctx->mu.
+static int32_t igd_build_dev(gtgpu_ctx* ctx, uint64_t n_files, uint32_t n_chroms, uint64_t total, const uint32_t* t_chr,
+                             const uint32_t* t_start, const uint32_t* t_end, const uint32_t* t_file, gtgpu_igd** out_igd) {
     cudaStream_t st = ctx->stream;
     gtgpu_igd* g = new gtgpu_igd();
     g->ctx = ctx;
@@ -368,30 +474,16 @@ static int32_t igd_build_one(gtgpu_ctx* ctx, uint64_t n_files, const uint64_t* f
         ~Guard() { if (g) gtgpu_igd_free(g); }
     } guard{g};
 
-    // ---- 1. records to the device; pooled order = stable sort by (chromosome, start) --------------------------------
+    // ---- 1. pooled order = stable sort by (chromosome, start) -------------------------------------------------------
     // ties keep (file, insertion) order = the order Igd::add saw them (igd.rs:285-301); records Igd::add drops get the
     // key n_chroms, land behind the last chromosome and are cut off
     TempPool tp;
-    uint32_t *t_chr, *t_start, *t_end, *t_file, *t_key, *t_off;
-    uint64_t* t_fo;
-    GT_TRY(tp.get(total, &t_chr));
-    GT_TRY(tp.get(total, &t_start));
-    GT_TRY(tp.get(total, &t_end));
-    GT_TRY(tp.get(total, &t_file));
+    uint32_t *t_key, *t_off;
     GT_TRY(tp.get(total, &t_key));
     GT_TRY(tp.get(n_chroms + 2, &t_off));
-    GT_TRY(tp.get(n_files + 1, &t_fo));
-    if (total) {
-        GT_CUDA(cudaMemcpyAsync(t_chr, chr, total * 4, cudaMemcpyHostToDevice, st));
-        GT_CUDA(cudaMemcpyAsync(t_start, start, total * 4, cudaMemcpyHostToDevice, st));
-        GT_CUDA(cudaMemcpyAsync(t_end, end, total * 4, cudaMemcpyHostToDevice, st));
-    }
-    GT_CUDA(cudaMemcpyAsync(t_fo, file_offsets, (n_files + 1) * 8, cudaMemcpyHostToDevice, st));
-    GT_CUDA(cudaStreamSynchronize(st));  // the caller's arrays may be pageable
     PermSorter pooled;
     GT_TRY(pooled.init(ctx, total));
     if (total) {
-        GT_TRY(launch_fill_set_ids(ctx, n_files, t_fo, t_file));
         igd_chrom_keys_kernel<<<grid_for(ctx, total), 256, 0, st>>>(total, n_chroms, t_chr, t_start, t_end, t_key);
         ctx->launches++;
         GT_TRY(pooled.pass(t_start, 0));

@@ -614,8 +614,8 @@ int32_t gunzip_locked(gtgpu_ctx* ctx, uint64_t n_members, const uint8_t* gz, con
 
 // gzip members -> device text (SC_GZ_OUT); a text that does not fit in device memory is reported as such
 int32_t inflate_whole_locked(gtgpu_ctx* ctx, uint64_t n_members, const uint8_t* gz, const uint64_t* member_offsets, const std::string& who,
-                             uint8_t** d_text, uint64_t* n_text) {
-    const int32_t s = gunzip_locked(ctx, n_members, gz, member_offsets, nullptr, d_text, n_text);
+                             uint8_t** d_text, uint64_t* n_text, uint64_t* out_member_offsets) {
+    const int32_t s = gunzip_locked(ctx, n_members, gz, member_offsets, out_member_offsets, d_text, n_text);
     if (s == GTGPU_ERR_NOMEM)
         return fail(s, who + ": the inflated text does not fit in device memory (gzip input is inflated whole before it is parsed): " +
                            gtgpu_last_error());

@@ -27,7 +27,21 @@ namespace gtgpu {
 
 constexpr int INGEST_CHUNK = 64;  // bytes per thread in the newline passes
 
-__global__ void ingest_count_newlines_kernel(uint64_t n_bytes, const char* __restrict__ text, uint32_t* __restrict__ counts) {
+// first index of the sorted array a[0, n) whose value is >= key
+__device__ __forceinline__ uint32_t lower_bound_u32(const uint32_t* __restrict__ a, uint32_t n, uint32_t key) {
+    uint32_t lo = 0, hi = n;
+    while (lo < hi) {
+        const uint32_t mid = (lo + hi) >> 1;
+        if (a[mid] < key) lo = mid + 1;
+        else hi = mid;
+    }
+    return lo;
+}
+
+// Line breaks: every '\n', and (for a text of several files) the byte in front of a file start p that no '\n' precedes, so that a
+// file's last line ends with the file.  fstart: n_fstart sorted window-relative file starts in (0, n_bytes), or none.
+__global__ void ingest_count_newlines_kernel(uint64_t n_bytes, const char* __restrict__ text, uint32_t* __restrict__ counts,
+                                             const uint32_t* __restrict__ fstart, uint32_t n_fstart) {
     const uint64_t n_chunks = (n_bytes + INGEST_CHUNK - 1) / INGEST_CHUNK;
     const uint64_t stride = (uint64_t)gridDim.x * blockDim.x;
     for (uint64_t c = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x; c < n_chunks; c += stride) {
@@ -48,19 +62,26 @@ __global__ void ingest_count_newlines_kernel(uint64_t n_bytes, const char* __res
         } else {
             for (uint64_t i = a; i < b; ++i) k += text[i] == '\n';
         }
+        if (n_fstart)  // breaks at bytes i in [a, b) in front of a file start i + 1
+            for (uint32_t j = lower_bound_u32(fstart, n_fstart, (uint32_t)a + 1); j < n_fstart && fstart[j] <= b; ++j)
+                k += text[fstart[j] - 1] != '\n';
         counts[c] = k;
     }
 }
 
 __global__ void ingest_newline_positions_kernel(uint64_t n_bytes, const char* __restrict__ text, const uint32_t* __restrict__ rank,
-                                                uint32_t* __restrict__ nl_pos) {
+                                                uint32_t* __restrict__ nl_pos, const uint32_t* __restrict__ fstart, uint32_t n_fstart) {
     const uint64_t n_chunks = (n_bytes + INGEST_CHUNK - 1) / INGEST_CHUNK;
     const uint64_t stride = (uint64_t)gridDim.x * blockDim.x;
     for (uint64_t c = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x; c < n_chunks; c += stride) {
         const uint64_t a = c * INGEST_CHUNK, b = min(a + INGEST_CHUNK, n_bytes);
         uint32_t r = rank[c];
-        for (uint64_t i = a; i < b; ++i)
-            if (text[i] == '\n') nl_pos[r++] = (uint32_t)i;
+        uint32_t j = n_fstart ? lower_bound_u32(fstart, n_fstart, (uint32_t)a + 1) : 0;
+        for (uint64_t i = a; i < b; ++i) {
+            const bool at_file_start = j < n_fstart && fstart[j] == i + 1;
+            if (at_file_start) ++j;
+            if (text[i] == '\n' || at_file_start) nl_pos[r++] = (uint32_t)i;
+        }
     }
 }
 
@@ -88,19 +109,42 @@ __device__ bool has_prefix(const char* __restrict__ t, uint32_t a, uint32_t b, c
     return true;
 }
 
-// status per line: 0 = skipped (comment / header), 1 = region, 2 = malformed
+// status per line: 0 = skipped (comment / header), 1 = region, 2 = malformed.
+// FILES (a text of several BED files back to back, files.file_offsets in bytes of the whole text): a file start is a line start
+// even without a '\n' in front of it (the newline passes put a break there), the header rule applies to the first line of every
+// file, chromosome names are not looked up but carried as (FNV-1a hash, window offset, length) for the caller's name discovery,
+// and chr[li] receives the line's file index.  files.first_line[f] gets the text-wide index of file f's first line.
+template <bool FILES>
 __global__ void ingest_parse_lines_kernel(uint32_t n_lines, uint32_t n_newlines, uint64_t n_bytes, const char* __restrict__ text,
                                           const uint32_t* __restrict__ nl_pos, NameTable names, uint32_t* __restrict__ keep,
                                           uint32_t* __restrict__ chr, uint32_t* __restrict__ start, uint32_t* __restrict__ end,
-                                          uint32_t* __restrict__ first_bad_line) {
+                                          uint32_t* __restrict__ first_bad_line, BedFilesView files) {
     const uint32_t stride = gridDim.x * blockDim.x;
     for (uint32_t li = blockIdx.x * blockDim.x + threadIdx.x; li < n_lines; li += stride) {
         uint32_t a = li ? nl_pos[li - 1] + 1 : 0;
         uint32_t b = li < n_newlines ? nl_pos[li] : (uint32_t)n_bytes;
+        bool nl_end = li < n_newlines;
+        if (FILES && nl_end && text[b] != '\n') {  // a break in front of a file start: the line ends with its file
+            ++b;
+            nl_end = false;
+        }
         // BufRead::lines strips "\n" and a "\r" right before it; a final line WITHOUT a newline keeps its '\r' (the reference then
         // fails to parse the field, and so do we)
-        if (li < n_newlines && b > a && text[b - 1] == '\r') --b;
+        if (nl_end && b > a && text[b - 1] == '\r') --b;
         uint32_t k = 0, c = GTGPU_UNKNOWN_CHROM, s = 0, e = 0;
+        bool first = li == 0;
+        if (FILES) {  // the line's file: the last one that starts at or before it (empty files start where the next one does)
+            const unsigned long long pos = files.byte0 + a;
+            uint64_t lo = 0, hi = files.n_files;
+            while (hi - lo > 1) {
+                const uint64_t mid = (lo + hi) >> 1;
+                if (files.file_offsets[mid] <= pos) lo = mid;
+                else hi = mid;
+            }
+            c = (uint32_t)lo;
+            first = files.file_offsets[lo] == pos;
+            if (first) files.first_line[lo] = files.line0 + li;
+        }
         if (has_prefix(text, a, b, "browser", 7) || has_prefix(text, a, b, "track", 5) || has_prefix(text, a, b, "#", 1)) {
             k = 0;
         } else {
@@ -113,7 +157,7 @@ __global__ void ingest_parse_lines_kernel(uint32_t n_lines, uint32_t n_newlines,
             while (t3 < b && text[t3] != '\t') ++t3;
             const bool three = t1 < b && t2 < b;  // at least two tabs = three parts
             const bool s_ok = three && parse_u32_field(text, t1 + 1, t2, s);
-            if (li == 0 && three && !s_ok) {
+            if (first && three && !s_ok) {
                 k = 0;  // a column-header first row without '#' (region_set.rs:118-131)
             } else if (!s_ok || !parse_u32_field(text, t2 + 1, t3, e)) {
                 k = 2;
@@ -121,17 +165,23 @@ __global__ void ingest_parse_lines_kernel(uint32_t n_lines, uint32_t n_newlines,
                 k = 1;
                 unsigned long long h = 1469598103934665603ull;  // FNV-1a 64
                 for (uint32_t i = a; i < t1; ++i) h = (h ^ (unsigned char)text[i]) * 1099511628211ull;
-                uint32_t lo = 0, hi = names.n_names;
-                while (lo < hi) {
-                    const uint32_t mid = (lo + hi) >> 1;
-                    if (names.hash[mid] < h) lo = mid + 1;
-                    else hi = mid;
-                }
-                for (; lo < names.n_names && names.hash[lo] == h; ++lo) {  // equal hashes: compare the bytes
-                    const uint32_t id = names.hash_id[lo], na = names.offsets[id], nb = names.offsets[id + 1];
-                    bool same = nb - na == t1 - a;
-                    for (uint32_t i = 0; same && i < nb - na; ++i) same = names.blob[na + i] == text[a + i];
-                    if (same) { c = id; break; }
+                if (FILES) {
+                    files.name_hash[li] = h ? h : 1;  // 0 marks an empty slot of the name table
+                    files.name_off[li] = a;
+                    files.name_len[li] = t1 - a;
+                } else {
+                    uint32_t lo = 0, hi = names.n_names;
+                    while (lo < hi) {
+                        const uint32_t mid = (lo + hi) >> 1;
+                        if (names.hash[mid] < h) lo = mid + 1;
+                        else hi = mid;
+                    }
+                    for (; lo < names.n_names && names.hash[lo] == h; ++lo) {  // equal hashes: compare the bytes
+                        const uint32_t id = names.hash_id[lo], na = names.offsets[id], nb = names.offsets[id + 1];
+                        bool same = nb - na == t1 - a;
+                        for (uint32_t i = 0; same && i < nb - na; ++i) same = names.blob[na + i] == text[a + i];
+                        if (same) { c = id; break; }
+                    }
                 }
             }
         }
@@ -448,19 +498,18 @@ int32_t upload_name_table(gtgpu_ctx* ctx, uint32_t n_names, const char* names, c
     return GTGPU_OK;
 }
 
-// The fragment front end shared by tokenize_fragment_file and the scoring entry points: newline positions, one thread per
-// line, compaction of the kept lines.  d_text: 0 < n_bytes < 0xFFFFFFF0 bytes of device text, 16-byte aligned.
-int32_t parse_fragments_locked(gtgpu_ctx* ctx, const char* d_text, uint64_t n_bytes, const NameTable& nt, FragMode mode,
-                               FragParse* out) {
+// Line breaks of device text (every '\n', and the breaks in front of the d_fstart file starts): *d_nl (scratch SC_IN3_END) gets
+// the n_breaks break positions, *n_lines counts the lines (the last one may end without a break).  Synchronises the ctx stream.
+static int32_t line_breaks_locked(gtgpu_ctx* ctx, const char* d_text, uint64_t n_bytes, const uint32_t* d_fstart, uint32_t n_fstart,
+                                  uint32_t* n_breaks, uint32_t* n_lines, uint32_t** d_nl) {
     cudaStream_t st = ctx->stream;
-    uint32_t *d_counts, *d_crank, *d_nl;
+    uint32_t *d_counts, *d_crank;
     void* d_tmp;
     const uint64_t n_chunks = (n_bytes + INGEST_CHUNK - 1) / INGEST_CHUNK;
     GT_TRY(ctx->scratch_get(SC_COUNTS, n_chunks * 4 + 4, (void**)&d_counts));
     GT_TRY(ctx->scratch_get(SC_IN3_CHR, n_chunks * 4 + 4, (void**)&d_crank));
-    // ---- lines -------------------------------------------------------------------------------------------------------------
     GT_TRY(ctx->scratch_get(SC_IN3_START, exclusive_scan_temp_bytes(n_chunks, 4), &d_tmp));
-    ingest_count_newlines_kernel<<<igrid(ctx, n_chunks), 256, 0, st>>>(n_bytes, d_text, d_counts);
+    ingest_count_newlines_kernel<<<igrid(ctx, n_chunks), 256, 0, st>>>(n_bytes, d_text, d_counts, d_fstart, n_fstart);
     ctx->launches++;
     GT_TRY(exclusive_scan<uint32_t>(ctx, d_counts, d_crank, n_chunks, d_tmp));
     uint32_t last[2];
@@ -469,11 +518,23 @@ int32_t parse_fragments_locked(gtgpu_ctx* ctx, const char* d_text, uint64_t n_by
     char last_byte = 0;  // read back from the device: with device-resident text there is no host copy
     GT_CUDA(cudaMemcpyAsync(&last_byte, d_text + n_bytes - 1, 1, cudaMemcpyDeviceToHost, st));
     GT_CUDA(cudaStreamSynchronize(st));
-    const uint32_t n_newlines = last[0] + last[1];
-    const uint32_t n_lines = n_newlines + (last_byte != '\n' ? 1u : 0u);
-    GT_TRY(ctx->scratch_get(SC_IN3_END, (size_t)n_newlines * 4 + 4, (void**)&d_nl));
-    ingest_newline_positions_kernel<<<igrid(ctx, n_chunks), 256, 0, st>>>(n_bytes, d_text, d_crank, d_nl);
+    *n_breaks = last[0] + last[1];
+    *n_lines = *n_breaks + (last_byte != '\n' ? 1u : 0u);
+    GT_TRY(ctx->scratch_get(SC_IN3_END, (size_t)*n_breaks * 4 + 4, (void**)d_nl));
+    ingest_newline_positions_kernel<<<igrid(ctx, n_chunks), 256, 0, st>>>(n_bytes, d_text, d_crank, *d_nl, d_fstart, n_fstart);
     ctx->launches++;
+    return GTGPU_OK;
+}
+
+// The fragment front end shared by tokenize_fragment_file and the scoring entry points: newline positions, one thread per
+// line, compaction of the kept lines.  d_text: 0 < n_bytes < 0xFFFFFFF0 bytes of device text, 16-byte aligned.
+int32_t parse_fragments_locked(gtgpu_ctx* ctx, const char* d_text, uint64_t n_bytes, const NameTable& nt, FragMode mode,
+                               FragParse* out) {
+    cudaStream_t st = ctx->stream;
+    uint32_t* d_nl;
+    void* d_tmp;
+    uint32_t n_newlines, n_lines;
+    GT_TRY(line_breaks_locked(ctx, d_text, n_bytes, nullptr, 0, &n_newlines, &n_lines, &d_nl));
     // ---- parse + compact ---------------------------------------------------------------------------------------------------
     const bool bc = mode != FRAG_SCORE_MATRIX;
     const size_t lb = (size_t)n_lines * 4 + 8;
@@ -711,7 +772,7 @@ static int32_t parse_bed_locked(gtgpu_ctx* ctx, const char* host_text, const cha
 
     // ---- 1. newline positions ---------------------------------------------------------------------------------------------
     GT_TRY(ctx->scratch_get(SC_IN3_START, exclusive_scan_temp_bytes(n_chunks, 4), &d_tmp));
-    ingest_count_newlines_kernel<<<igrid(ctx, n_chunks), 256, 0, st>>>(n_bytes, d_text, d_counts);
+    ingest_count_newlines_kernel<<<igrid(ctx, n_chunks), 256, 0, st>>>(n_bytes, d_text, d_counts, nullptr, 0);
     ctx->launches++;
     GT_TRY(exclusive_scan<uint32_t>(ctx, d_counts, d_crank, n_chunks, d_tmp));
     uint32_t last[2];
@@ -723,7 +784,7 @@ static int32_t parse_bed_locked(gtgpu_ctx* ctx, const char* host_text, const cha
     const uint32_t n_newlines = last[0] + last[1];
     const uint32_t n_lines = n_newlines + (last_byte != '\n' ? 1u : 0u);
     GT_TRY(ctx->scratch_get(SC_IN3_END, (size_t)n_newlines * 4 + 4, (void**)&d_nl));
-    ingest_newline_positions_kernel<<<igrid(ctx, n_chunks), 256, 0, st>>>(n_bytes, d_text, d_crank, d_nl);
+    ingest_newline_positions_kernel<<<igrid(ctx, n_chunks), 256, 0, st>>>(n_bytes, d_text, d_crank, d_nl, nullptr, 0);
     ctx->launches++;
 
     // ---- 2. parse, 3. compact ---------------------------------------------------------------------------------------------
@@ -744,8 +805,8 @@ static int32_t parse_bed_locked(gtgpu_ctx* ctx, const char* host_text, const cha
     const uint32_t init[2] = {0xFFFFFFFFu, 0u};
     GT_CUDA(cudaMemcpyAsync(d_flags, init, 8, cudaMemcpyHostToDevice, st));
     NameTable nt{d_blob, d_noff, d_hash, d_hid, n_names};
-    ingest_parse_lines_kernel<<<igrid(ctx, n_lines), 256, 0, st>>>(n_lines, n_newlines, n_bytes, d_text, d_nl, nt, d_keep, p_chr, p_start,
-                                                                   p_end, d_flags);
+    ingest_parse_lines_kernel<false><<<igrid(ctx, n_lines), 256, 0, st>>>(n_lines, n_newlines, n_bytes, d_text, d_nl, nt, d_keep, p_chr,
+                                                                          p_start, p_end, d_flags, BedFilesView{});
     ctx->launches++;
     GT_TRY(exclusive_scan<uint32_t>(ctx, d_keep, d_pos, n_lines, d_tmp));
     ingest_compact_kernel<<<igrid(ctx, n_lines), 256, 0, st>>>(n_lines, d_keep, d_pos, p_chr, p_start, p_end, o_chr, o_start, o_end);
@@ -986,6 +1047,271 @@ int32_t tokenize_fragments_file_locked(gtgpu_index* ix, const char* host_text, c
     *out_n_barcodes = n_barcodes;
     *out_barcode_offsets = std::move(offs);
     *out_ids = std::move(ids);
+    return GTGPU_OK;
+}
+
+// ---- the BED files of an IGD database: region lines of many files, chromosome names discovered on the device ------------------
+// Name table: open addressing on the 64-bit FNV-1a hash of a chromosome name, NAME_SLOTS slots (an assembly names 25 to ~1e5
+// contigs).  Every record finds or claims its name's slot and lowers the slot's first appearance to its own record index; that
+// head copies the name's bytes to an arena, every later record compares its bytes with them (a 64-bit hash collision would merge
+// two names).  A record's chr column holds its slot until the last window, when the slots are numbered in first-appearance order.
+constexpr uint32_t NAME_SLOTS = 1u << 19, MAX_NAMES = NAME_SLOTS / 2;
+
+__global__ void ingest_name_insert_kernel(uint32_t n, const unsigned long long* __restrict__ h, unsigned long long* keys,
+                                          uint32_t* first, uint32_t* __restrict__ slot_of, uint32_t base, uint32_t* __restrict__ full) {
+    const uint32_t stride = gridDim.x * blockDim.x;
+    for (uint32_t k = blockIdx.x * blockDim.x + threadIdx.x; k < n; k += stride) {
+        const unsigned long long key = h[k];
+        uint32_t slot = (uint32_t)((key * 0x9E3779B97F4A7C15ull) >> 32) & (NAME_SLOTS - 1), probes = 0;
+        for (;;) {
+            unsigned long long prev = keys[slot];  // a set key never changes: only an empty slot needs the CAS
+            if (prev == 0ull) prev = atomicCAS(keys + slot, 0ull, key);
+            if (prev == 0ull || prev == key) break;
+            slot = (slot + 1) & (NAME_SLOTS - 1);
+            if (++probes == NAME_SLOTS) {  // more names than slots: reported, never spun on
+                atomicOr(full, 1u);
+                slot = NAME_SLOTS;
+                break;
+            }
+        }
+        // consecutive records mostly share a chromosome: the first lane of each group of equal slots lowers the first appearance
+        const unsigned same = __match_any_sync(__activemask(), slot);
+        if (slot < NAME_SLOTS && (threadIdx.x & 31) == (unsigned)(__ffs(same) - 1) && first[slot] > base + k) atomicMin(first + slot, base + k);
+        slot_of[k] = slot;
+    }
+}
+
+// counters[0] = arena bytes claimed so far, counters[1] = distinct names
+__global__ void ingest_name_heads_kernel(uint32_t n, uint32_t base, const uint32_t* __restrict__ slot_of, const uint32_t* __restrict__ first,
+                                         const uint32_t* __restrict__ len, uint32_t* __restrict__ nlen, unsigned long long* __restrict__ soff,
+                                         unsigned long long* __restrict__ counters) {
+    const uint32_t stride = gridDim.x * blockDim.x;
+    for (uint32_t k = blockIdx.x * blockDim.x + threadIdx.x; k < n; k += stride) {
+        const uint32_t s = slot_of[k];
+        if (s < NAME_SLOTS && first[s] == base + k) {
+            nlen[s] = len[k];
+            soff[s] = atomicAdd(counters, (unsigned long long)len[k]);
+            atomicAdd(counters + 1, 1ull);
+        }
+    }
+}
+
+__global__ void ingest_name_claim_kernel(uint32_t n, uint32_t base, const char* __restrict__ text, const uint32_t* __restrict__ slot_of,
+                                         const uint32_t* __restrict__ first, const uint32_t* __restrict__ off, const uint32_t* __restrict__ len,
+                                         const unsigned long long* __restrict__ soff, char* __restrict__ arena) {
+    const uint32_t stride = gridDim.x * blockDim.x;
+    for (uint32_t k = blockIdx.x * blockDim.x + threadIdx.x; k < n; k += stride) {
+        const uint32_t s = slot_of[k];
+        if (first[s] != base + k) continue;
+        for (uint32_t i = 0; i < len[k]; ++i) arena[soff[s] + i] = text[off[k] + i];
+    }
+}
+
+__global__ void ingest_name_check_kernel(uint32_t n, uint32_t base, const char* __restrict__ text, const uint32_t* __restrict__ slot_of,
+                                         const uint32_t* __restrict__ first, const uint32_t* __restrict__ off, const uint32_t* __restrict__ len,
+                                         const uint32_t* __restrict__ nlen, const unsigned long long* __restrict__ soff,
+                                         const char* __restrict__ arena, uint32_t* __restrict__ collision) {
+    const uint32_t stride = gridDim.x * blockDim.x;
+    for (uint32_t k = blockIdx.x * blockDim.x + threadIdx.x; k < n; k += stride) {
+        const uint32_t s = slot_of[k];
+        if (first[s] == base + k) continue;
+        const uint64_t p = soff[s];
+        bool same = nlen[s] == len[k];
+        for (uint32_t i = 0; same && i < len[k]; ++i) same = arena[p + i] == text[off[k] + i];
+        if (!same) *collision = 1;
+    }
+}
+
+__global__ void ingest_name_ids_kernel(uint64_t n, const uint32_t* __restrict__ id_of_slot, uint32_t* __restrict__ chr) {
+    const uint64_t stride = (uint64_t)gridDim.x * blockDim.x;
+    for (uint64_t g = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x; g < n; g += stride) chr[g] = id_of_slot[chr[g]];
+}
+
+// records are in file order: file f's records start at the first record whose file is >= f
+__global__ void ingest_file_record_offsets_kernel(uint64_t n_files, const uint32_t* __restrict__ file, uint64_t n,
+                                                  unsigned long long* __restrict__ out) {
+    const uint64_t stride = (uint64_t)gridDim.x * blockDim.x;
+    for (uint64_t f = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x; f <= n_files; f += stride) {
+        uint64_t lo = 0, hi = n;
+        while (lo < hi) {
+            const uint64_t mid = (lo + hi) >> 1;
+            if (file[mid] < f) lo = mid + 1;
+            else hi = mid;
+        }
+        out[f] = lo;
+    }
+}
+
+int32_t parse_bed_files_locked(gtgpu_ctx* ctx, const char* host_text, const char* dev_text, uint64_t n_files, const uint64_t* file_offsets,
+                               const std::string& who, BedFilesRecords* out) {
+    cudaStream_t st = ctx->stream;
+    const uint64_t n_bytes = file_offsets[n_files];
+    DevMem d_fo, d_first_line, d_fs, keys, first, soff, nlen, arena, counters;
+    GT_TRY(d_fo.reserve((n_files + 1) * 8, 0, st));
+    GT_TRY(d_first_line.reserve(std::max<uint64_t>(n_files, 1) * 8, 0, st));
+    GT_TRY(keys.reserve((size_t)NAME_SLOTS * 8, 0, st));
+    GT_TRY(first.reserve((size_t)NAME_SLOTS * 4, 0, st));
+    GT_TRY(soff.reserve((size_t)NAME_SLOTS * 8, 0, st));
+    GT_TRY(nlen.reserve((size_t)NAME_SLOTS * 4, 0, st));
+    GT_TRY(counters.reserve(32, 0, st));
+    GT_CUDA(cudaMemcpyAsync(d_fo.ptr, file_offsets, (n_files + 1) * 8, cudaMemcpyHostToDevice, st));
+    GT_CUDA(cudaMemsetAsync(keys.ptr, 0, (size_t)NAME_SLOTS * 8, st));
+    GT_CUDA(cudaMemsetAsync(first.ptr, 0xFF, (size_t)NAME_SLOTS * 4, st));
+    GT_CUDA(cudaMemsetAsync(counters.ptr, 0, 32, st));
+    GT_CUDA(cudaStreamSynchronize(st));  // file_offsets is the caller's
+    unsigned long long* cnt = (unsigned long long*)counters.ptr;  // [0] arena bytes, [1] names, [2] table full / collision flags
+    uint32_t* d_full = (uint32_t*)(cnt + 2);
+    uint64_t used = 0;
+    BedFilesRecords& r = *out;
+    r.n = 0;
+    std::vector<uint32_t> fs;  // the window's file starts that are not its first byte (window-relative)
+    GT_TRY(for_each_window(ctx, host_text, dev_text, n_bytes, who,
+                           [&](const char* d, uint64_t nb, uint64_t byte0, uint64_t line0, uint32_t* n_lines_out) -> int32_t {
+        fs.clear();
+        for (const uint64_t* f = std::upper_bound(file_offsets, file_offsets + n_files + 1, byte0);
+             f < file_offsets + n_files + 1 && *f < byte0 + nb; ++f)
+            if (fs.empty() || fs.back() != *f - byte0) fs.push_back((uint32_t)(*f - byte0));
+        if (!fs.empty()) {
+            GT_TRY(d_fs.reserve(fs.size() * 4, 0, st));
+            GT_CUDA(cudaMemcpyAsync(d_fs.ptr, fs.data(), fs.size() * 4, cudaMemcpyHostToDevice, st));
+        }
+        uint32_t *d_nl, n_breaks, n_lines;
+        GT_TRY(line_breaks_locked(ctx, d, nb, d_fs.u32(), (uint32_t)fs.size(), &n_breaks, &n_lines, &d_nl));
+        *n_lines_out = n_lines;
+        // ---- parse + compact (the compaction of the fragment parse carries the same six columns) --------------------------------
+        const size_t lb = (size_t)n_lines * 4 + 8;
+        uint32_t *d_keep, *d_pos, *p_file, *p_start, *p_end, *p_off, *p_len, *o_file, *o_start, *o_end, *o_off, *o_len, *d_flags;
+        unsigned long long *p_h, *o_h;
+        void* d_tmp;
+        GT_TRY(ctx->scratch_get(SC_IN3_START, exclusive_scan_temp_bytes(n_lines, 4), &d_tmp));
+        GT_TRY(ctx->scratch_get(SC_ING_0, lb, (void**)&d_keep));
+        GT_TRY(ctx->scratch_get(SC_ING_1, lb, (void**)&d_pos));
+        GT_TRY(ctx->scratch_get(SC_IN2_CHR, lb, (void**)&p_file));
+        GT_TRY(ctx->scratch_get(SC_IN2_START, lb, (void**)&p_start));
+        GT_TRY(ctx->scratch_get(SC_IN2_END, lb, (void**)&p_end));
+        GT_TRY(ctx->scratch_get(SC_CHR, lb, (void**)&o_file));
+        GT_TRY(ctx->scratch_get(SC_START, lb, (void**)&o_start));
+        GT_TRY(ctx->scratch_get(SC_END, lb, (void**)&o_end));
+        GT_TRY(ctx->scratch_get(SC_ING_2, lb * 2, (void**)&p_h));
+        GT_TRY(ctx->scratch_get(SC_ING_3, lb, (void**)&p_off));
+        GT_TRY(ctx->scratch_get(SC_ING_4, lb, (void**)&p_len));
+        GT_TRY(ctx->scratch_get(SC_ING_5, lb * 2, (void**)&o_h));
+        GT_TRY(ctx->scratch_get(SC_ING_6, lb, (void**)&o_off));
+        GT_TRY(ctx->scratch_get(SC_ING_7, lb, (void**)&o_len));
+        GT_TRY(ctx->scratch_get(SC_MISC, 64, (void**)&d_flags));  // [0] first malformed line, [1] name collision
+        const uint32_t init[2] = {0xFFFFFFFFu, 0u};
+        GT_CUDA(cudaMemcpyAsync(d_flags, init, 8, cudaMemcpyHostToDevice, st));
+        BedFilesView fv;
+        fv.file_offsets = (const unsigned long long*)d_fo.ptr;
+        fv.n_files = n_files;
+        fv.byte0 = byte0;
+        fv.line0 = line0;
+        fv.first_line = (unsigned long long*)d_first_line.ptr;
+        fv.name_hash = p_h;
+        fv.name_off = p_off;
+        fv.name_len = p_len;
+        ingest_parse_lines_kernel<true><<<igrid(ctx, n_lines), 256, 0, st>>>(n_lines, n_breaks, nb, d, d_nl, NameTable{}, d_keep, p_file,
+                                                                             p_start, p_end, d_flags, fv);
+        ctx->launches++;
+        GT_TRY(exclusive_scan<uint32_t>(ctx, d_keep, d_pos, n_lines, d_tmp));
+        ingest_compact_fragments_kernel<<<igrid(ctx, n_lines), 256, 0, st>>>(n_lines, d_keep, d_pos, p_file, p_start, p_end, p_h, p_off,
+                                                                             p_len, o_file, o_start, o_end, o_h, o_off, o_len);
+        ctx->launches++;
+        uint32_t tail[3];
+        GT_CUDA(cudaMemcpyAsync(&tail[0], d_pos + n_lines - 1, 4, cudaMemcpyDeviceToHost, st));
+        GT_CUDA(cudaMemcpyAsync(&tail[1], d_keep + n_lines - 1, 4, cudaMemcpyDeviceToHost, st));
+        GT_CUDA(cudaMemcpyAsync(&tail[2], d_flags, 4, cudaMemcpyDeviceToHost, st));
+        GT_CUDA(cudaStreamSynchronize(st));
+        if (tail[2] != 0xFFFFFFFFu) {  // the file of the first malformed line and the line's number in that file
+            const uint32_t li = tail[2];
+            uint32_t a = 0;
+            if (li) GT_CUDA(cudaMemcpy(&a, d_nl + li - 1, 4, cudaMemcpyDeviceToHost));
+            const uint64_t pos = byte0 + (li ? a + 1ull : 0ull);
+            const uint64_t f = (uint64_t)(std::upper_bound(file_offsets, file_offsets + n_files, pos) - file_offsets) - 1;
+            unsigned long long fl = 0;
+            GT_CUDA(cudaMemcpy(&fl, (unsigned long long*)d_first_line.ptr + f, 8, cudaMemcpyDeviceToHost));
+            return fail(GTGPU_ERR_INVALID, who + ": file " + std::to_string(f) + ", line " + std::to_string(line0 + li - fl + 1) +
+                                               ": cannot parse start / end position (RegionParseError)");
+        }
+        const uint32_t nw = tail[0] + tail[1];
+        if (nw == 0) return GTGPU_OK;
+        if (r.n + nw >= 0xFFFFFFFFull) return fail(GTGPU_ERR_UNSUPPORTED, who + ": 2^32 - 1 region lines or more");
+        // ---- append the window's records; their names go through the table -------------------------------------------------
+        const uint32_t base = (uint32_t)r.n;
+        const size_t need = (size_t)(r.n + nw) * 4, have = (size_t)r.n * 4;
+        for (DevMem* m : {&r.chr, &r.start, &r.end, &r.file}) GT_TRY(m->reserve(need, have, st));
+        GT_CUDA(cudaMemcpyAsync(r.start.u32() + base, o_start, (size_t)nw * 4, cudaMemcpyDeviceToDevice, st));
+        GT_CUDA(cudaMemcpyAsync(r.end.u32() + base, o_end, (size_t)nw * 4, cudaMemcpyDeviceToDevice, st));
+        GT_CUDA(cudaMemcpyAsync(r.file.u32() + base, o_file, (size_t)nw * 4, cudaMemcpyDeviceToDevice, st));
+        uint32_t* slot_of = r.chr.u32() + base;
+        ingest_name_insert_kernel<<<igrid(ctx, nw), 256, 0, st>>>(nw, o_h, (unsigned long long*)keys.ptr, first.u32(), slot_of, base, d_full);
+        ingest_name_heads_kernel<<<igrid(ctx, nw), 256, 0, st>>>(nw, base, slot_of, first.u32(), o_len, nlen.u32(),
+                                                                 (unsigned long long*)soff.ptr, cnt);
+        ctx->launches += 2;
+        unsigned long long c[3];
+        GT_CUDA(cudaMemcpyAsync(c, cnt, 24, cudaMemcpyDeviceToHost, st));
+        GT_CUDA(cudaStreamSynchronize(st));
+        if ((uint32_t)c[2] || c[1] > MAX_NAMES)
+            return fail(GTGPU_ERR_UNSUPPORTED, who + ": more than " + std::to_string(MAX_NAMES) + " distinct chromosome names");
+        GT_TRY(arena.reserve(c[0] + 1, used, st));
+        ingest_name_claim_kernel<<<igrid(ctx, nw), 256, 0, st>>>(nw, base, d, slot_of, first.u32(), o_off, o_len,
+                                                                 (const unsigned long long*)soff.ptr, (char*)arena.ptr);
+        ingest_name_check_kernel<<<igrid(ctx, nw), 256, 0, st>>>(nw, base, d, slot_of, first.u32(), o_off, o_len, nlen.u32(),
+                                                                 (const unsigned long long*)soff.ptr, (const char*)arena.ptr, d_flags + 1);
+        ctx->launches += 2;
+        uint32_t collision = 0;
+        GT_CUDA(cudaMemcpyAsync(&collision, d_flags + 1, 4, cudaMemcpyDeviceToHost, st));
+        GT_CUDA(cudaStreamSynchronize(st));  // the window's text may be overwritten after this
+        if (collision) return fail(GTGPU_ERR_UNSUPPORTED, who + ": two chromosome names share a 64-bit hash; use gtgpu_igd_build");
+        used = c[0];
+        r.n += nw;
+        return GTGPU_OK;
+    }));
+    // ---- every file has a region line; records per file ---------------------------------------------------------------------
+    r.file_offsets.assign(n_files + 1, 0);
+    if (n_files) {
+        DevMem roff;
+        GT_TRY(roff.reserve((n_files + 1) * 8, 0, st));
+        if (r.n) {
+            ingest_file_record_offsets_kernel<<<igrid(ctx, n_files + 1), 256, 0, st>>>(n_files, r.file.u32(), r.n,
+                                                                                      (unsigned long long*)roff.ptr);
+            ctx->launches++;
+            GT_CUDA(cudaMemcpyAsync(r.file_offsets.data(), roff.ptr, (n_files + 1) * 8, cudaMemcpyDeviceToHost, st));
+            GT_CUDA(cudaStreamSynchronize(st));
+        }
+        for (uint64_t f = 0; f < n_files; ++f)
+            if (r.file_offsets[f + 1] == r.file_offsets[f])
+                return fail(GTGPU_ERR_INVALID, who + ": file " + std::to_string(f) + ": Corrupted file. 0 regions found");
+    }
+    // ---- chromosome ids in first-appearance order; the records' slots become ids ----------------------------------------------
+    std::vector<unsigned long long> h_keys(NAME_SLOTS), h_soff(NAME_SLOTS);
+    std::vector<uint32_t> h_first(NAME_SLOTS), h_nlen(NAME_SLOTS), id_of_slot(NAME_SLOTS, 0), slots;
+    std::string arena_bytes(used, '\0');
+    GT_CUDA(cudaMemcpyAsync(h_keys.data(), keys.ptr, (size_t)NAME_SLOTS * 8, cudaMemcpyDeviceToHost, st));
+    GT_CUDA(cudaMemcpyAsync(h_soff.data(), soff.ptr, (size_t)NAME_SLOTS * 8, cudaMemcpyDeviceToHost, st));
+    GT_CUDA(cudaMemcpyAsync(h_first.data(), first.ptr, (size_t)NAME_SLOTS * 4, cudaMemcpyDeviceToHost, st));
+    GT_CUDA(cudaMemcpyAsync(h_nlen.data(), nlen.ptr, (size_t)NAME_SLOTS * 4, cudaMemcpyDeviceToHost, st));
+    if (used) GT_CUDA(cudaMemcpyAsync(&arena_bytes[0], arena.ptr, used, cudaMemcpyDeviceToHost, st));
+    GT_CUDA(cudaStreamSynchronize(st));
+    for (uint32_t s = 0; s < NAME_SLOTS; ++s)
+        if (h_keys[s]) slots.push_back(s);
+    std::sort(slots.begin(), slots.end(), [&](uint32_t a, uint32_t b) { return h_first[a] < h_first[b]; });
+    r.names.clear();
+    r.name_offsets.assign(1, 0);
+    for (uint32_t id = 0; id < slots.size(); ++id) {
+        id_of_slot[slots[id]] = id;
+        r.names.append(arena_bytes, h_soff[slots[id]], h_nlen[slots[id]]);
+        r.name_offsets.push_back(r.names.size());
+    }
+    if (r.n) {
+        DevMem d_ids;
+        GT_TRY(d_ids.reserve((size_t)NAME_SLOTS * 4, 0, st));
+        GT_CUDA(cudaMemcpyAsync(d_ids.ptr, id_of_slot.data(), (size_t)NAME_SLOTS * 4, cudaMemcpyHostToDevice, st));
+        ingest_name_ids_kernel<<<igrid(ctx, r.n), 256, 0, st>>>(r.n, d_ids.u32(), r.chr.u32());
+        ctx->launches++;
+        GT_CUDA(cudaGetLastError());
+        GT_CUDA(cudaStreamSynchronize(st));  // id_of_slot is pageable
+    }
     return GTGPU_OK;
 }
 

@@ -619,14 +619,21 @@ std::vector<uint32_t> Tokenizer::encode(const std::vector<Region>& regions) cons
 // A `.gz` input made of many gzip members (bgzip / BGZF, or concatenated gzips) is inflated on the device, one warp per
 // member, and parsed there; a single-member stream is sequential, so it stays with zlib on the host (get_dynamic_reader's
 // MultiGzDecoder semantics either way: the text is the concatenation of the members).
-static bool gz_members_for_device(const std::string& path, std::string& raw, std::vector<uint64_t>& members) {
-    if (!(path.size() >= 3 && path.compare(path.size() - 3, 3, ".gz") == 0)) return false;
+static bool ends_with_gz(const std::string& path) { return path.size() >= 3 && path.compare(path.size() - 3, 3, ".gz") == 0; }
+
+// the file's bytes as stored (no decompression)
+static void read_raw_bytes(const std::string& path, std::string& raw) {
     std::ifstream f(path, std::ios::binary | std::ios::ate);
     if (!f) throw Error("Failed to open file: \"" + path + "\"");
     const std::streamsize size = f.tellg();
     f.seekg(0);
     raw.resize((size_t)std::max<std::streamsize>(size, 0));
     if (size > 0 && !f.read(&raw[0], size)) throw Error("Failed to read file: \"" + path + "\"");
+}
+
+static bool gz_members_for_device(const std::string& path, std::string& raw, std::vector<uint64_t>& members) {
+    if (!ends_with_gz(path)) return false;
+    read_raw_bytes(path, raw);
     uint64_t n = 0;
     gtgpu_gzip_members((const uint8_t*)raw.data(), raw.size(), 0, nullptr, &n);  // count only
     if (n < 16) return false;
@@ -1137,6 +1144,88 @@ std::unique_ptr<Igd> Igd::from_igd_file(std::shared_ptr<Device> dev, const std::
                           &g->igd_),
           "gtgpu_igd_build");
     return g;
+}
+
+std::unique_ptr<Igd> Igd::from_bed_files(std::shared_ptr<Device> dev, const std::vector<std::string>& paths) {
+    std::unique_ptr<Igd> g(new Igd());
+    g->dev_ = dev;
+    g->n_files_ = paths.size();
+    uint32_t n_chroms = 0;
+    PinnedResult names, name_offsets;
+    int32_t status;
+    const char* fn;
+    if (!paths.empty() && std::all_of(paths.begin(), paths.end(), ends_with_gz)) {
+        // one-member .bed.gz files are the common case: every member of every file is inflated on the device in parallel
+        std::string gz, raw;
+        std::vector<uint64_t> members{0}, file_members{0}, m;
+        for (const auto& p : paths) {
+            read_raw_bytes(p, raw);
+            uint64_t n = 0;
+            gtgpu_gzip_members((const uint8_t*)raw.data(), raw.size(), 0, nullptr, &n);  // count only
+            m.assign(n + 1, 0);
+            check(gtgpu_gzip_members((const uint8_t*)raw.data(), raw.size(), m.size(), m.data(), &n), "gtgpu_gzip_members");
+            for (uint64_t k = 1; k <= n; ++k) members.push_back(gz.size() + m[k]);
+            file_members.push_back(members.size() - 1);
+            gz += raw;
+        }
+        fn = "gtgpu_igd_build_bed_gz";
+        status = gtgpu_igd_build_bed_gz(dev->ctx(), paths.size(), file_members.data(), members.size() - 1, (const uint8_t*)gz.data(),
+                                        members.data(), &n_chroms, &names.buf, &name_offsets.buf, &g->igd_);
+    } else {
+        // the texts back to back; the library stages them to the device through its own pinned blocks
+        std::vector<uint64_t> file_offsets{0};
+        std::vector<std::string> inflated(paths.size());
+        for (size_t f = 0; f < paths.size(); ++f) {
+            uint64_t size = 0;
+            if (ends_with_gz(paths[f])) {
+                inflated[f] = read_file_bytes(paths[f]);
+                size = inflated[f].size();
+            } else {
+                std::ifstream in(paths[f], std::ios::binary | std::ios::ate);
+                if (!in) throw Error("Failed to open file: \"" + paths[f] + "\"");
+                size = (uint64_t)std::max<std::streamsize>(in.tellg(), 0);
+            }
+            file_offsets.push_back(file_offsets.back() + size);
+        }
+        std::unique_ptr<char[]> text(new char[std::max<uint64_t>(file_offsets.back(), 1)]);
+        for (size_t f = 0; f < paths.size(); ++f) {
+            char* dst = text.get() + file_offsets[f];
+            const uint64_t size = file_offsets[f + 1] - file_offsets[f];
+            if (ends_with_gz(paths[f])) {
+                memcpy(dst, inflated[f].data(), size);
+                std::string().swap(inflated[f]);
+            } else if (size) {
+                std::ifstream in(paths[f], std::ios::binary);
+                if (!in || !in.read(dst, (std::streamsize)size)) throw Error("Failed to read file: \"" + paths[f] + "\"");
+            }
+        }
+        fn = "gtgpu_igd_build_bed";
+        status = gtgpu_igd_build_bed(dev->ctx(), paths.size(), text.get(), file_offsets.data(), &n_chroms, &names.buf, &name_offsets.buf,
+                                     &g->igd_);
+    }
+    if (status != GTGPU_OK) {  // "file k" in the library's message becomes the file's path
+        std::string msg = gtgpu_last_error();
+        const size_t k = msg.find(": file ");
+        size_t b = k == std::string::npos ? k : k + 7;
+        if (b != std::string::npos) {
+            const size_t a = b;
+            while (b < msg.size() && isdigit((unsigned char)msg[b])) ++b;
+            if (b > a && std::stoull(msg.substr(a, b - a)) < paths.size())
+                msg = msg.substr(0, k) + ": \"" + paths[std::stoull(msg.substr(a, b - a))] + "\"" + msg.substr(b);
+        }
+        throw Error(std::string(fn) + ": " + msg);
+    }
+    const char* blob = (const char*)gtgpu_buf_data(names.buf);
+    const uint64_t* noff = (const uint64_t*)gtgpu_buf_data(name_offsets.buf);
+    for (uint32_t c = 0; c < n_chroms; ++c) g->cmap_.add(std::string(blob + noff[c], noff[c + 1] - noff[c]));
+    return g;
+}
+
+std::array<uint64_t, 4> Igd::info() const {
+    if (!igd_) throw Error("info needs a database Igd (not from_single_region_set)");
+    std::array<uint64_t, 4> a{};
+    check(gtgpu_igd_info(igd_, a.data()), "gtgpu_igd_info");
+    return a;
 }
 
 std::unique_ptr<Igd> Igd::from_single_region_set(std::shared_ptr<Device> dev, const RegionSet& subject) {

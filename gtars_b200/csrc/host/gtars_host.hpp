@@ -17,6 +17,7 @@
 #include <string>
 #include <unordered_map>
 #include <utility>
+#include <array>
 #include <vector>
 
 #include "../../../include/gtars_gpu.h"
@@ -263,6 +264,13 @@ class Igd {
     static void save_named_region_sets(const std::vector<std::pair<std::string, const RegionSet*>>& sets, const std::string& path,
                                        int32_t nbp = 16384);
     static std::unique_ptr<Igd> from_igd_file(std::shared_ptr<Device> dev, const std::string& path);
+    // Igd(RegionSet::from_file(p) for p in paths) with every file's text parsed on the device (gtgpu_igd_build_bed): when every
+    // path ends in ".gz" the gzip bytes go to the device inflater (gtgpu_igd_build_bed_gz), otherwise each file is read (".gz"
+    // inflated by zlib) and the texts go back to back.  Chromosome ids follow the names' first appearance in the files.  Errors
+    // name the file's path.
+    static std::unique_ptr<Igd> from_bed_files(std::shared_ptr<Device> dev, const std::vector<std::string>& paths);
+    // gtgpu_igd_info: n_files, records kept, device bytes, LUT shift (a database Igd only)
+    std::array<uint64_t, 4> info() const;
 
     // Igd::from_single_region_set (igd.rs:609-634): two-set overlap queries; the subject index is kept per record.
     static std::unique_ptr<Igd> from_single_region_set(std::shared_ptr<Device> dev, const RegionSet& subject);

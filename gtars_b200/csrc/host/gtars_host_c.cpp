@@ -303,6 +303,18 @@ int gth_igd_save_sets(uint64_t n, void** region_sets, const char** names, const 
 void* gth_igd_from_file(void* dev, const char* path) {
     return guard([&]() -> void* { return Igd::from_igd_file(*(std::shared_ptr<Device>*)dev, path).release(); }, nullptr);
 }
+void* gth_igd_from_bed_files(void* dev, uint64_t n, const char** paths) {
+    return guard([&]() -> void* {
+        return Igd::from_bed_files(*(std::shared_ptr<Device>*)dev, std::vector<std::string>(paths, paths + n)).release();
+    }, nullptr);
+}
+int gth_igd_info(void* g, uint64_t* out /* 4 */) {
+    return guard([&]() -> int {
+        auto a = ((Igd*)g)->info();
+        std::copy(a.begin(), a.end(), out);
+        return 0;
+    }, 1);
+}
 void gth_igd_free(void* g) { delete (Igd*)g; }
 uint64_t gth_igd_num_files(void* g) { return ((Igd*)g)->num_files(); }
 int gth_igd_count(void* g, uint64_t n_sets, void** region_sets, int32_t min_overlap, int pairwise, uint64_t* out) {

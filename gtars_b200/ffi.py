@@ -70,6 +70,8 @@ SIGNATURES = {
     "gtgpu_score_barcodes_text": (_i32, [_vp, _vp, _u64, _u32, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp]),
     "gtgpu_score_barcodes_gz": (_i32, [_vp, _u64, _vp, _vp, _u32, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp]),
     "gtgpu_igd_build": (_i32, [_vp, _u64, _vp, _u32, _vp, _vp, _vp, _vp]),
+    "gtgpu_igd_build_bed": (_i32, [_vp, _u64, _vp, _vp, _vp, _vp, _vp, _vp]),
+    "gtgpu_igd_build_bed_gz": (_i32, [_vp, _u64, _vp, _u64, _vp, _vp, _vp, _vp, _vp, _vp]),
     "gtgpu_igd_free": (_i32, [_vp]),
     "gtgpu_igd_info": (_i32, [_vp, _vp]),
     "gtgpu_igd_count_set_overlaps": (_i32, [_vp, _u64, _vp, _vp, _vp, _vp, _i32, _vp]),
@@ -560,6 +562,31 @@ class Igd:
         self.n_files = len(fo) - 1
         self._h = C.c_void_p()
         check(lib().gtgpu_igd_build(ctx._h, self.n_files, _p(fo), n_chroms, _p(chr), _p(start), _p(end), C.byref(self._h)))
+
+    @classmethod
+    def _from_bed(cls, ctx, n_files, call):
+        obj = cls.__new__(cls)
+        obj.ctx, obj.n_files, obj._h = ctx, n_files, C.c_void_p()
+        nc, hn, hno = C.c_uint32(0), C.c_void_p(), C.c_void_p()
+        check(call(C.byref(nc), C.byref(hn), C.byref(hno), C.byref(obj._h)))
+        names = _take(hn, dtype=np.uint8).tobytes()
+        no = _take(hno, dtype=np.uint64)
+        return obj, [names[int(a):int(b)].decode() for a, b in zip(no[:-1], no[1:])]
+
+    @classmethod
+    def from_bed_text(cls, ctx: Context, text, file_offsets):
+        """gtgpu_igd_build_bed: file f = text[file_offsets[f]:file_offsets[f + 1]], parsed on the device.  Returns (igd,
+        chromosome names in id order).  `text` may be a uint8 numpy array (a multi-GB text is not copied)."""
+        fo = _arr(file_offsets, np.uint64)
+        return cls._from_bed(ctx, len(fo) - 1, lambda *outs: lib().gtgpu_igd_build_bed(ctx._h, len(fo) - 1, _text_ptr(text), _p(fo), *outs))
+
+    @classmethod
+    def from_bed_gz(cls, ctx: Context, gz, file_members, member_offsets):
+        """gtgpu_igd_build_bed_gz: file f = gzip members [file_members[f], file_members[f + 1]) of `gz` (member_offsets as
+        gzip_members returns them), inflated and parsed on the device.  Returns (igd, chromosome names in id order)."""
+        fm, mo = _arr(file_members, np.uint64), _arr(member_offsets, np.uint64)
+        return cls._from_bed(ctx, len(fm) - 1, lambda *outs: lib().gtgpu_igd_build_bed_gz(ctx._h, len(fm) - 1, _p(fm), len(mo) - 1,
+                                                                                          _text_ptr(gz), _p(mo), *outs))
 
     def close(self):
         if getattr(self, "_h", None) and getattr(self.ctx, "_h", None):

@@ -345,6 +345,25 @@ int32_t gtgpu_score_barcodes(gtgpu_index* index, uint64_t n, const uint32_t* chr
  * Igd::add does (igd.rs:109-116).  chr ids must be < n_chroms. */
 int32_t gtgpu_igd_build(gtgpu_ctx* ctx, uint64_t n_files, const uint64_t* file_offsets, uint32_t n_chroms,
                         const uint32_t* chr, const uint32_t* start, const uint32_t* end, gtgpu_igd** out_igd);
+/* gtgpu_igd_build from the database's BED files, parsed on the device (Igd::from_named_region_sets over RegionSet::try_from of
+ * every file, gtars-core/src/models/region_set.rs:60-185): file f = text[file_offsets[f], file_offsets[f+1]) of any total
+ * size, or the gzip members [file_members[f], file_members[f+1]) of gz / member_offsets (as in gtgpu_gunzip; inflated whole into
+ * device memory, GTGPU_ERR_NOMEM when that text does not fit).  Every file follows the line rules of gtgpu_parse_bed: browser /
+ * track / '#' lines are skipped, a first line of the file whose second field is not a u32 is a header, every other line needs
+ * three tab-separated fields with u32 start and end.  A file's end ends its last line (a line never spans two files).  A region
+ * line that gtgpu_igd_build would drop (start >= end, or negative as int32) still counts as a region of its file.  Chromosome
+ * ids are the names' first-appearance order over the region lines (files in order, lines in file order); *out_n_chroms names
+ * come back as their bytes back to back (*out_chrom_names, u8) and n_chroms + 1 u64 offsets (*out_chrom_name_offsets): a
+ * caller maps query chromosomes through them.  Errors (GTGPU_ERR_INVALID, no IGD): a malformed line ("file k, line j", j
+ * 1-based within file k; reported before an empty file); a file without a region line ("file k: ... 0 regions found").
+ * Distinct names are found with 64-bit FNV-1a + a byte comparison: a true hash collision, more than 262 144 distinct names or
+ * 2^32 - 1 region lines give GTGPU_ERR_UNSUPPORTED.  The text is parsed in windows of about GTGPU_INGEST_WINDOW bytes (default
+ * 2 GiB) on the first device of a multi-device ctx; the shards of a group are then copied from there to their devices. */
+int32_t gtgpu_igd_build_bed(gtgpu_ctx* ctx, uint64_t n_files, const char* text, const uint64_t* file_offsets, uint32_t* out_n_chroms,
+                            gtgpu_buf** out_chrom_names, gtgpu_buf** out_chrom_name_offsets, gtgpu_igd** out_igd);
+int32_t gtgpu_igd_build_bed_gz(gtgpu_ctx* ctx, uint64_t n_files, const uint64_t* file_members, uint64_t n_members, const uint8_t* gz,
+                               const uint64_t* member_offsets, uint32_t* out_n_chroms, gtgpu_buf** out_chrom_names,
+                               gtgpu_buf** out_chrom_name_offsets, gtgpu_igd** out_igd);
 int32_t gtgpu_igd_free(gtgpu_igd* igd);
 /* info[0]=n_files, [1]=records kept, [2]=device bytes, [3]=lut shift */
 int32_t gtgpu_igd_info(const gtgpu_igd* igd, uint64_t info[4]);
