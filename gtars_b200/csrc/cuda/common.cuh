@@ -331,41 +331,70 @@ int32_t radix_group_values(gtgpu_ctx* ctx, uint64_t n_cap, const uint32_t* keys,
                            uint64_t* out_offsets, uint64_t* d_total);
 
 // ingest.cu / inflate.cu (the caller holds ctx->mu)
+// 64-bit FNV-1a of n bytes
+__host__ __device__ __forceinline__ unsigned long long fnv1a64(const char* p, uint32_t n) {
+    unsigned long long h = 1469598103934665603ull;
+    for (uint32_t i = 0; i < n; ++i) h = (h ^ (unsigned char)p[i]) * 1099511628211ull;
+    return h;
+}
 struct NameTable {
     const char* blob;             // names back to back
     const uint32_t* offsets;      // n_names + 1
     const unsigned long long* hash;  // FNV-1a of every name, sorted ascending
     const uint32_t* hash_id;      // name id of the k-th sorted hash
     uint32_t n_names;
+    const uint32_t* rank;         // lexicographic rank of every name (only when asked for)
+    // id of the name s[0, len) with FNV-1a hash h, or GTGPU_UNKNOWN_CHROM
+    __device__ uint32_t lookup(unsigned long long h, const char* __restrict__ s, uint32_t len) const {
+        uint32_t lo = 0, hi = n_names;
+        while (lo < hi) {
+            const uint32_t mid = (lo + hi) >> 1;
+            if (hash[mid] < h) lo = mid + 1;
+            else hi = mid;
+        }
+        for (; lo < n_names && hash[lo] == h; ++lo) {  // equal hashes: compare the bytes
+            const uint32_t id = hash_id[lo], na = offsets[id], nb = offsets[id + 1];
+            bool same = nb - na == len;
+            for (uint32_t i = 0; same && i < len; ++i) same = blob[na + i] == s[i];
+            if (same) return id;
+        }
+        return GTGPU_UNKNOWN_CHROM;
+    }
 };
+// the caller's chromosome names -> scratch SC_SET_ID; with_rank adds the names' lexicographic ranks (NameTable::rank)
+int32_t upload_name_table(gtgpu_ctx* ctx, uint32_t n_names, const char* names, const uint32_t* name_offsets, NameTable* out,
+                          bool with_rank = false);
 // What the BED line kernel needs to parse a text of several files back to back (ingest_parse_lines_kernel<true>).
 struct BedFilesView {
     const unsigned long long* file_offsets = nullptr;  // n_files + 1 byte offsets of the files in the whole text
     uint64_t n_files = 0;
     uint64_t byte0 = 0, line0 = 0;                     // the window's first byte and first line in the whole text
     unsigned long long* first_line = nullptr;          // [f] = text-wide index of file f's first line
-    unsigned long long* name_hash = nullptr;           // per line: FNV-1a of the chromosome name (never 0), its window
-    uint32_t *name_off = nullptr, *name_len = nullptr;  // offset and length
+    const uint32_t* fstart = nullptr;                  // the window's n_fstart file starts in (0, n_bytes), sorted
+    uint32_t n_fstart = 0;
 };
-// the caller's chromosome names -> scratch SC_SET_ID
-int32_t upload_name_table(gtgpu_ctx* ctx, uint32_t n_names, const char* names, const uint32_t* name_offsets, NameTable* out);
-// What the fragment parse checks and carries: tokenize_fragment_file needs fields 1 and 2 as u32 and the barcode;
-// Fragment::from_str (scoring) needs field 4 as well, and the count matrix has no use for the barcode.
-enum FragMode { FRAG_TOKENIZE = 0, FRAG_SCORE_MATRIX = 1, FRAG_SCORE_BARCODES = 2 };
-struct FragParse {
+// The line formats of the device text parsers; each has its own line kernel, the front end around it is shared.
+// BED_LINES: gtgpu_parse_bed's rules, names looked up in the name table.  BED_FILE_LINES: the same per file of a BedFilesView,
+// chr = the line's file index, and the chromosome name carried as a key.  Fragments: tokenize_fragment_file needs fields 1
+// and 2 as u32 and the barcode (the key); Fragment::from_str (scoring) needs field 4 as well, and the count matrix has no use
+// for the barcode.
+enum LineFormat { BED_LINES, BED_FILE_LINES, FRAG_TOKENIZE, FRAG_SCORE_MATRIX, FRAG_SCORE_BARCODES };
+struct ParsedLines {
     uint32_t n_lines = 0;
     uint32_t bad_line = 0xFFFFFFFFu;  // 0-based index of the first malformed line of the text, or none
-    uint32_t n = 0;                   // fragments (0 when a line was malformed)
+    uint32_t n = 0;                   // kept lines (0 when a line was malformed)
     uint32_t *chr = nullptr, *start = nullptr, *end = nullptr;  // scratch SC_CHR / SC_START / SC_END
-    unsigned long long* h = nullptr;                             // barcode hash, byte offset and length (not for the matrix)
-    uint32_t *bo = nullptr, *bl = nullptr;
-    uint32_t *free0 = nullptr, *free1 = nullptr, *free2 = nullptr;  // line-sized scratch the caller may reuse
-    void* tmp = nullptr;                                           // scan temp for line-sized arrays
-    uint32_t* flags = nullptr;                                     // device words [1..3], zeroed for the caller
+    unsigned long long* h = nullptr;  // per kept line the key's FNV-1a hash (never 0), byte offset and length in the text
+    uint32_t *bo = nullptr, *bl = nullptr;  // (BED_FILE_LINES, FRAG_TOKENIZE, FRAG_SCORE_BARCODES only)
+    const uint32_t* breaks = nullptr;       // the line break positions (scratch SC_IN3_END): line i > 0 starts at breaks[i - 1] + 1
+    uint32_t* free[5] = {};  // line-sized scratch the caller may reuse (SC_ING_0, SC_ING_1, SC_IN2_CHR, SC_IN2_START, SC_IN2_END)
+    void* tmp = nullptr;     // scan temp for line-sized arrays (scratch SC_IN3_START)
+    uint32_t* flags = nullptr;  // device words [1..3], zeroed for the caller (scratch SC_MISC)
 };
-// d_text: 0 < n_bytes < 0xFFFFFFF0 bytes of device text, 16-byte aligned.  Synchronises the ctx stream.
-int32_t parse_fragments_locked(gtgpu_ctx* ctx, const char* d_text, uint64_t n_bytes, const NameTable& nt, FragMode mode,
-                               FragParse* out);
+// The line front end: line breaks, the format's one-thread-per-line kernel, compaction of the kept lines.  d_text: 0 < n_bytes
+// < 0xFFFFFFF0 bytes of device text, 16-byte aligned; files only for BED_FILE_LINES.  Synchronises the ctx stream.
+int32_t parse_lines_locked(gtgpu_ctx* ctx, const char* d_text, uint64_t n_bytes, LineFormat fmt, const NameTable& nt,
+                           const BedFilesView& files, ParsedLines* out);
 // A device buffer owned by one call, grown while keeping its first `keep` bytes.
 struct DevMem {
     void* ptr = nullptr;
@@ -378,22 +407,27 @@ struct DevMem {
     void swap(DevMem& o) { std::swap(ptr, o.ptr); std::swap(cap, o.cap); }
     uint32_t* u32() const { return static_cast<uint32_t*>(ptr); }
 };
-// Barcodes of one fragment file over all its windows: dense ids in first-appearance order among the kept barcodes.  keep_all
-// (tokenization) keeps every barcode; otherwise (scoring) only those seen on a chromosome of the name table are kept.
-// record_spans keeps each barcode's first byte offset in the file for finish()'s spans.  who / array_entry name the caller and
-// its array entry point in error messages.  chr / start / end / bc hold every fragment of the file once finish() has run.
-struct FragBarcodeTable {
+// The keys of one text over all its windows (barcodes of a fragment file, chromosome names of BED files): dense ids in
+// first-appearance order among the kept keys.  keep_all keeps every key; otherwise only those seen on a line whose chr is in
+// the name table are kept.  At most max_keys distinct keys are allowed.  record_spans keeps each key's first byte offset in
+// the text for finish()'s spans.  who / array_entry name the caller and its array entry point in error messages; key / keys
+// name one key and the keys in them.  chr / start / end hold the parsed columns of every kept line, id the key's
+// first-appearance index per line, and after finish() the key's dense id (0 for a line of a dropped key).
+struct KeyTable {
     const bool keep_all, record_spans;
-    const std::string who, array_entry;
-    DevMem chr, start, end, fidx, known, hlen, first_byte, bc;
-    DevMem keys, first, soff, arena;
+    const uint64_t max_keys;
+    const std::string who, array_entry, key, keys;
+    DevMem chr, start, end, id;                                // per line
+    DevMem hash, first, soff, klen, known, first_byte, arena;  // per slot (hash 0 = empty), and the keys' bytes
     uint64_t n = 0, distinct = 0, cap = 0, used = 0;
-    FragBarcodeTable(bool keep_all_, bool record_spans_, std::string who_, std::string array_entry_)
-        : keep_all(keep_all_), record_spans(record_spans_), who(std::move(who_)), array_entry(std::move(array_entry_)) {}
-    // byte0: the window's offset in the file
-    int32_t add_window(gtgpu_ctx* ctx, const char* d_text, uint64_t byte0, const FragParse& fp, uint32_t n_names);
+    KeyTable(bool keep_all_, bool record_spans_, uint64_t max_keys_, std::string who_, std::string array_entry_, std::string key_,
+             std::string keys_)
+        : keep_all(keep_all_), record_spans(record_spans_), max_keys(max_keys_), who(std::move(who_)),
+          array_entry(std::move(array_entry_)), key(std::move(key_)), keys(std::move(keys_)) {}
+    // byte0: the window's offset in the text; pl carries keys (h / bo / bl)
+    int32_t add_window(gtgpu_ctx* ctx, const char* d_text, uint64_t byte0, const ParsedLines& pl, uint32_t n_names);
     // With out_spans (needs record_spans): n_kept (first byte, length) u32 pairs, and out_names / out_name_offsets are untouched.
-    // Otherwise *out_names: the kept barcodes' bytes back to back (elem_size 1); *out_name_offsets: n_kept + 1 u64 offsets into them.
+    // Otherwise *out_names: the kept keys' bytes back to back (elem_size 1); *out_name_offsets: n_kept + 1 u64 offsets into them.
     int32_t finish(gtgpu_ctx* ctx, uint32_t* n_kept, BufPtr* out_names, BufPtr* out_name_offsets, BufPtr* out_spans = nullptr);
 };
 // A fragment text of any size in windows that end right after a '\n' (about GTGPU_INGEST_WINDOW bytes, default 2 GiB).  fn gets
@@ -422,13 +456,13 @@ int32_t tokenize_fragments_file_locked(gtgpu_index* ix, const char* host_text, c
 // The region lines of n_files BED files back to back (file f = text[file_offsets[f], file_offsets[f + 1]), any total size),
 // parsed on the device in windows: line rules of gtgpu_parse_bed per file, chromosome names discovered in first-appearance order.
 // On success chr / start / end / file hold the n records in file order (chr = dense name id), file_offsets the files' record
-// offsets (n_files + 1), names / name_offsets the chromosome names in id order.  The caller holds ctx->mu.
+// offsets (n_files + 1), names / name_offsets the n_names chromosome names in id order.  The caller holds ctx->mu.
 struct BedFilesRecords {
     DevMem chr, start, end, file;
     uint64_t n = 0;
     std::vector<uint64_t> file_offsets;
-    std::string names;
-    std::vector<uint64_t> name_offsets;
+    uint32_t n_names = 0;
+    BufPtr names, name_offsets;
 };
 int32_t parse_bed_files_locked(gtgpu_ctx* ctx, const char* host_text, const char* dev_text, uint64_t n_files, const uint64_t* file_offsets,
                                const std::string& who, BedFilesRecords* out);

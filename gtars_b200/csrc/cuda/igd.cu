@@ -361,12 +361,7 @@ extern "C" int32_t gtgpu_igd_build(gtgpu_ctx* ctx, uint64_t n_files, const uint6
 // device with cudaMemcpyAsync by the builder of gtgpu_igd_build (igd_records_to_device).
 static int32_t igd_build_parsed(gtgpu_ctx* ctx, uint64_t n_files, BedFilesRecords& r, uint32_t* out_n_chroms, gtgpu_buf** out_names,
                                 gtgpu_buf** out_name_offsets, gtgpu_igd** out_igd) {
-    const uint32_t n_chroms = (uint32_t)(r.name_offsets.size() - 1);
-    BufPtr names, offsets;
-    GT_TRY(buf_new(ctx, r.names.size(), 1, &names));
-    GT_TRY(buf_new(ctx, n_chroms + 1, 8, &offsets));
-    if (!r.names.empty()) memcpy(names->block.ptr, r.names.data(), r.names.size());
-    memcpy(offsets->block.ptr, r.name_offsets.data(), (n_chroms + 1) * 8);
+    const uint32_t n_chroms = r.n_names;
     gtgpu_igd* g = nullptr;
     if (ctx->peers.size() > 1) {
         GT_TRY(igd_build_group(ctx, n_files, r.file_offsets.data(), n_chroms, r.chr.u32(), r.start.u32(), r.end.u32(), &g));
@@ -377,8 +372,8 @@ static int32_t igd_build_parsed(gtgpu_ctx* ctx, uint64_t n_files, BedFilesRecord
         GT_TRY(igd_build_dev(ctx, n_files, n_chroms, r.n, r.chr.u32(), r.start.u32(), r.end.u32(), r.file.u32(), &g));
     }
     *out_n_chroms = n_chroms;
-    *out_names = names.release();
-    *out_name_offsets = offsets.release();
+    *out_names = r.names.release();
+    *out_name_offsets = r.name_offsets.release();
     *out_igd = g;
     return GTGPU_OK;
 }

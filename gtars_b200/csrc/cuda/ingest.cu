@@ -109,15 +109,22 @@ __device__ bool has_prefix(const char* __restrict__ t, uint32_t a, uint32_t b, c
     return true;
 }
 
+// The columns a line kernel writes per line of its window (keep = the line is kept), and the compaction writes per kept line.
+// h / bo / bl: the line's key (FNV-1a hash, never 0; byte offset and length in the window), null for a format without keys.
+struct LineCols {
+    uint32_t *keep, *chr, *start, *end;
+    unsigned long long* h;
+    uint32_t *bo, *bl;
+};
+
 // status per line: 0 = skipped (comment / header), 1 = region, 2 = malformed.
 // FILES (a text of several BED files back to back, files.file_offsets in bytes of the whole text): a file start is a line start
 // even without a '\n' in front of it (the newline passes put a break there), the header rule applies to the first line of every
-// file, chromosome names are not looked up but carried as (FNV-1a hash, window offset, length) for the caller's name discovery,
-// and chr[li] receives the line's file index.  files.first_line[f] gets the text-wide index of file f's first line.
+// file, chromosome names are not looked up but carried as the line's key for the caller's name discovery, and chr[li] receives
+// the line's file index.  files.first_line[f] gets the text-wide index of file f's first line.
 template <bool FILES>
 __global__ void ingest_parse_lines_kernel(uint32_t n_lines, uint32_t n_newlines, uint64_t n_bytes, const char* __restrict__ text,
-                                          const uint32_t* __restrict__ nl_pos, NameTable names, uint32_t* __restrict__ keep,
-                                          uint32_t* __restrict__ chr, uint32_t* __restrict__ start, uint32_t* __restrict__ end,
+                                          const uint32_t* __restrict__ nl_pos, NameTable names, LineCols o,
                                           uint32_t* __restrict__ first_bad_line, BedFilesView files) {
     const uint32_t stride = gridDim.x * blockDim.x;
     for (uint32_t li = blockIdx.x * blockDim.x + threadIdx.x; li < n_lines; li += stride) {
@@ -163,48 +170,22 @@ __global__ void ingest_parse_lines_kernel(uint32_t n_lines, uint32_t n_newlines,
                 k = 2;
             } else {
                 k = 1;
-                unsigned long long h = 1469598103934665603ull;  // FNV-1a 64
-                for (uint32_t i = a; i < t1; ++i) h = (h ^ (unsigned char)text[i]) * 1099511628211ull;
+                const unsigned long long h = fnv1a64(text + a, t1 - a);
                 if (FILES) {
-                    files.name_hash[li] = h ? h : 1;  // 0 marks an empty slot of the name table
-                    files.name_off[li] = a;
-                    files.name_len[li] = t1 - a;
+                    o.h[li] = h ? h : 1;  // 0 marks an empty slot of the key table
+                    o.bo[li] = a;
+                    o.bl[li] = t1 - a;
                 } else {
-                    uint32_t lo = 0, hi = names.n_names;
-                    while (lo < hi) {
-                        const uint32_t mid = (lo + hi) >> 1;
-                        if (names.hash[mid] < h) lo = mid + 1;
-                        else hi = mid;
-                    }
-                    for (; lo < names.n_names && names.hash[lo] == h; ++lo) {  // equal hashes: compare the bytes
-                        const uint32_t id = names.hash_id[lo], na = names.offsets[id], nb = names.offsets[id + 1];
-                        bool same = nb - na == t1 - a;
-                        for (uint32_t i = 0; same && i < nb - na; ++i) same = names.blob[na + i] == text[a + i];
-                        if (same) { c = id; break; }
-                    }
+                    c = names.lookup(h, text + a, t1 - a);
                 }
             }
         }
         if (k == 2) atomicMin(first_bad_line, li);
-        keep[li] = k == 1;
-        chr[li] = c;
-        start[li] = s;
-        end[li] = e;
+        o.keep[li] = k == 1;
+        o.chr[li] = c;
+        o.start[li] = s;
+        o.end[li] = e;
     }
-}
-
-__global__ void ingest_compact_kernel(uint32_t n_lines, const uint32_t* __restrict__ keep, const uint32_t* __restrict__ pos,
-                                      const uint32_t* __restrict__ chr, const uint32_t* __restrict__ start,
-                                      const uint32_t* __restrict__ end, uint32_t* __restrict__ o_chr, uint32_t* __restrict__ o_start,
-                                      uint32_t* __restrict__ o_end) {
-    const uint32_t stride = gridDim.x * blockDim.x;
-    for (uint32_t i = blockIdx.x * blockDim.x + threadIdx.x; i < n_lines; i += stride)
-        if (keep[i]) {
-            const uint32_t p = pos[i];
-            o_chr[p] = chr[i];
-            o_start[p] = start[i];
-            o_end[p] = end[i];
-        }
 }
 
 __device__ __forceinline__ uint32_t rank_of(const uint32_t* __restrict__ name_rank, uint32_t n_names, uint32_t c) {
@@ -252,17 +233,15 @@ __device__ __forceinline__ bool is_space(char c) { return c == ' ' || (c >= '\t'
 // parse has no use for it and skips the hashing.
 template <bool SUPPORT, bool BARCODE>
 __global__ void ingest_parse_fragments_kernel(uint32_t n_lines, uint32_t n_newlines, uint64_t n_bytes, const char* __restrict__ text,
-                                              const uint32_t* __restrict__ nl_pos, NameTable names, uint32_t* __restrict__ keep,
-                                              uint32_t* __restrict__ chr, uint32_t* __restrict__ start, uint32_t* __restrict__ end,
-                                              unsigned long long* __restrict__ bc_hash, uint32_t* __restrict__ bc_off,
-                                              uint32_t* __restrict__ bc_len, uint32_t* __restrict__ first_bad_line) {
+                                              const uint32_t* __restrict__ nl_pos, NameTable names, LineCols o,
+                                              uint32_t* __restrict__ first_bad_line) {
     const uint32_t stride = gridDim.x * blockDim.x;
     for (uint32_t li = blockIdx.x * blockDim.x + threadIdx.x; li < n_lines; li += stride) {
         uint32_t a = li ? nl_pos[li - 1] + 1 : 0;
         uint32_t b = li < n_newlines ? nl_pos[li] : (uint32_t)n_bytes;
         if (li < n_newlines && b > a && text[b - 1] == '\r') --b;  // only a '\r' in front of a '\n' is part of the line ending
         uint32_t k = 0, c = GTGPU_UNKNOWN_CHROM, s = 0, e = 0, bo = 0, bl = 0, sup = 0;
-        unsigned long long h = 1469598103934665603ull;
+        unsigned long long h = 1;
         if (!(b > a && text[a] == '#')) {
             uint32_t fa[5], fb[5], nf = 0, p = a;
             while (nf < 5) {
@@ -277,188 +256,201 @@ __global__ void ingest_parse_fragments_kernel(uint32_t n_lines, uint32_t n_newli
                 k = 2;
             } else {
                 k = 1;
-                unsigned long long hc = 1469598103934665603ull;
-                for (uint32_t i = fa[0]; i < fb[0]; ++i) hc = (hc ^ (unsigned char)text[i]) * 1099511628211ull;
-                uint32_t lo = 0, hi = names.n_names;
-                while (lo < hi) {
-                    const uint32_t mid = (lo + hi) >> 1;
-                    if (names.hash[mid] < hc) lo = mid + 1;
-                    else hi = mid;
-                }
-                for (; lo < names.n_names && names.hash[lo] == hc; ++lo) {
-                    const uint32_t id = names.hash_id[lo], na = names.offsets[id], nb = names.offsets[id + 1];
-                    bool same = nb - na == fb[0] - fa[0];
-                    for (uint32_t i = 0; same && i < nb - na; ++i) same = names.blob[na + i] == text[fa[0] + i];
-                    if (same) { c = id; break; }
-                }
+                c = names.lookup(fnv1a64(text + fa[0], fb[0] - fa[0]), text + fa[0], fb[0] - fa[0]);
                 if (BARCODE) {
                     bo = fa[3];
                     bl = fb[3] - fa[3];
-                    for (uint32_t i = fa[3]; i < fb[3]; ++i) h = (h ^ (unsigned char)text[i]) * 1099511628211ull;
-                    if (h == 0) h = 1;  // 0 marks an empty slot of the barcode table
+                    h = fnv1a64(text + bo, bl);
+                    if (h == 0) h = 1;  // 0 marks an empty slot of the key table
                 }
             }
         }
         if (k == 2) atomicMin(first_bad_line, li);
-        keep[li] = k == 1;
-        chr[li] = c;
-        start[li] = s;
-        end[li] = e;
+        o.keep[li] = k == 1;
+        o.chr[li] = c;
+        o.start[li] = s;
+        o.end[li] = e;
         if (BARCODE) {
-            bc_hash[li] = h;
-            bc_off[li] = bo;
-            bc_len[li] = bl;
+            o.h[li] = h;
+            o.bo[li] = bo;
+            o.bl[li] = bl;
         }
     }
 }
 
-__global__ void ingest_compact_fragments_kernel(uint32_t n_lines, const uint32_t* __restrict__ keep, const uint32_t* __restrict__ pos,
-                                                const uint32_t* __restrict__ chr, const uint32_t* __restrict__ start,
-                                                const uint32_t* __restrict__ end, const unsigned long long* __restrict__ h,
-                                                const uint32_t* __restrict__ bo, const uint32_t* __restrict__ bl,
-                                                uint32_t* __restrict__ o_chr, uint32_t* __restrict__ o_start, uint32_t* __restrict__ o_end,
-                                                unsigned long long* __restrict__ o_h, uint32_t* __restrict__ o_bo, uint32_t* __restrict__ o_bl) {
+__global__ void ingest_compact_lines_kernel(uint32_t n_lines, const uint32_t* __restrict__ pos, LineCols p, LineCols o) {
     const uint32_t stride = gridDim.x * blockDim.x;
     for (uint32_t i = blockIdx.x * blockDim.x + threadIdx.x; i < n_lines; i += stride)
-        if (keep[i]) {
-            const uint32_t p = pos[i];
-            o_chr[p] = chr[i];
-            o_start[p] = start[i];
-            o_end[p] = end[i];
-            if (o_h) {  // uniform per launch: the count-matrix parse carries no barcodes
-                o_h[p] = h[i];
-                o_bo[p] = bo[i];
-                o_bl[p] = bl[i];
+        if (p.keep[i]) {
+            const uint32_t q = pos[i];
+            o.chr[q] = p.chr[i];
+            o.start[q] = p.start[i];
+            o.end[q] = p.end[i];
+            if (o.h) {  // uniform per launch: only some formats carry keys
+                o.h[q] = p.h[i];
+                o.bo[q] = p.bo[i];
+                o.bl[q] = p.bl[i];
             }
         }
 }
 
-// Barcode table (open addressing on the 64-bit hash): every fragment finds or claims its barcode's slot and lowers the
-// slot's first-appearance index to its own position, base + k (base = fragments of the file before this window).
-__global__ void ingest_barcode_insert_kernel(uint32_t n, const unsigned long long* __restrict__ h, uint32_t mask,
-                                             unsigned long long* __restrict__ keys, uint32_t* __restrict__ first,
-                                             uint32_t* __restrict__ slot_of, uint32_t base) {
+// ---- the key table (KeyTable): open addressing on the 64-bit key hash, one table over all windows of a text -------------------
+// A window's lines are numbered text-wide (base + k), so a slot's first-appearance index is the text-wide index of the key's
+// first line.  Per line the table keeps that index (id); per slot the key's byte length, its offset in the arena (the window
+// that first sees a key copies its bytes there, because the text of a plain-text window leaves the device with it), "seen on
+// a chromosome of the name table" (known, when not every key is kept) and, when asked for, its first byte offset in the text.
+struct KeySlots {
+    unsigned long long *hash, *soff, *first_byte;
+    uint32_t *first, *klen, *known;
+};
+
+__device__ __forceinline__ uint32_t key_home(unsigned long long key, uint32_t mask) {
+    return (uint32_t)((key * 0x9E3779B97F4A7C15ull) >> 32) & mask;
+}
+
+// every line finds or claims its key's slot (slot_of[k]; mask + 1 when the table is full) and lowers the slot's first appearance
+__global__ void ingest_key_insert_kernel(uint32_t n, const unsigned long long* __restrict__ h, uint32_t mask, unsigned long long* hash,
+                                         uint32_t* first, uint32_t* __restrict__ slot_of, uint32_t base, uint32_t* __restrict__ full) {
     const uint32_t stride = gridDim.x * blockDim.x;
     for (uint32_t k = blockIdx.x * blockDim.x + threadIdx.x; k < n; k += stride) {
         const unsigned long long key = h[k];
-        uint32_t slot = (uint32_t)((key * 0x9E3779B97F4A7C15ull) >> 32) & mask;
+        uint32_t slot = key_home(key, mask), probes = 0;
         for (;;) {
-            const unsigned long long prev = atomicCAS(keys + slot, 0ull, key);
+            unsigned long long prev = hash[slot];  // a set key never changes: only an empty slot needs the CAS
+            if (prev == 0ull) prev = atomicCAS(hash + slot, 0ull, key);
             if (prev == 0ull || prev == key) break;
             slot = (slot + 1) & mask;
+            if (++probes > mask) {  // more keys than slots: reported, never spun on
+                atomicOr(full, 1u);
+                slot = mask + 1;
+                break;
+            }
         }
-        atomicMin(first + slot, base + k);
+        // consecutive lines often share a key: the first lane of each group of equal slots lowers the first appearance
+        const unsigned same = __match_any_sync(__activemask(), slot);
+        if (slot <= mask && (threadIdx.x & 31) == (unsigned)(__ffs(same) - 1) && first[slot] > base + k) atomicMin(first + slot, base + k);
         slot_of[k] = slot;
     }
 }
 
-// ---- the barcode table of the fragment-text entry points: one table over all windows of a file ------------------------------
-// A window's fragments are numbered file-wide (base + k), so a slot's first-appearance index is the file-wide index of the
-// barcode's first fragment.  Per fragment the table keeps fidx (that index), per barcode (at its first fragment g) hlen[g]
-// (its byte length), known[g] (seen on a chromosome of the name table) and, when asked for, first_byte[g] (the file offset of
-// its first occurrence); the bytes go to an arena in the window that first sees the barcode, in first-appearance order,
-// because the text of a plain-text window leaves the device with it.
-__global__ void ingest_barcode_rehash_kernel(uint64_t old_cap, const unsigned long long* __restrict__ okeys,
-                                             const uint32_t* __restrict__ ofirst, const unsigned long long* __restrict__ osoff,
-                                             uint32_t mask, unsigned long long* __restrict__ keys, uint32_t* __restrict__ first,
-                                             unsigned long long* __restrict__ soff) {
+__global__ void ingest_key_rehash_kernel(uint64_t old_cap, KeySlots o, uint32_t mask, KeySlots t) {
     const uint64_t stride = (uint64_t)gridDim.x * blockDim.x;
     for (uint64_t s = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x; s < old_cap; s += stride) {
-        const unsigned long long key = okeys[s];
+        const unsigned long long key = o.hash[s];
         if (!key) continue;
-        uint32_t slot = (uint32_t)((key * 0x9E3779B97F4A7C15ull) >> 32) & mask;
-        while (atomicCAS(keys + slot, 0ull, key) != 0ull) slot = (slot + 1) & mask;  // keys are distinct
-        first[slot] = ofirst[s];
-        soff[slot] = osoff[s];
+        uint32_t slot = key_home(key, mask);
+        while (atomicCAS(t.hash + slot, 0ull, key) != 0ull) slot = (slot + 1) & mask;  // keys are distinct
+        t.first[slot] = o.first[s];
+        t.soff[slot] = o.soff[s];
+        t.klen[slot] = o.klen[s];
+        if (t.known) t.known[slot] = o.known[s];
+        if (t.first_byte) t.first_byte[slot] = o.first_byte[s];
     }
 }
 
-__global__ void ingest_barcode_window_heads_kernel(uint32_t n, uint32_t base, const uint32_t* __restrict__ slot_of,
-                                                   const uint32_t* __restrict__ first, const uint32_t* __restrict__ chr,
-                                                   const uint32_t* __restrict__ bl, uint32_t n_names, uint32_t* __restrict__ fidx,
-                                                   uint32_t* __restrict__ hlen, uint32_t* __restrict__ known, uint32_t* __restrict__ n_new) {
+// per line its key's first appearance; per key first seen in this window its length (wlen, 0 for other lines, for the arena
+// scan); known keys are marked; n_new counts the keys first seen here
+__global__ void ingest_key_heads_kernel(uint32_t n, uint32_t base, const uint32_t* __restrict__ slot_of, const uint32_t* __restrict__ first,
+                                        const uint32_t* __restrict__ chr, const uint32_t* __restrict__ bl, uint32_t n_names, uint32_t mask,
+                                        uint32_t* __restrict__ id, uint32_t* __restrict__ klen, uint32_t* __restrict__ known,
+                                        uint32_t* __restrict__ wlen, uint32_t* __restrict__ n_new) {
     const uint32_t stride = gridDim.x * blockDim.x;
     for (uint32_t k = blockIdx.x * blockDim.x + threadIdx.x; k < n; k += stride) {
-        const uint32_t f = first[slot_of[k]], g = base + k;
+        const uint32_t s = slot_of[k], g = base + k;
+        const bool in_table = s <= mask;  // the lines of a full table are reported by the insert and skipped here
+        const uint32_t f = in_table ? first[s] : 0xFFFFFFFFu;
         const bool head = f == g;
-        fidx[g] = f;
-        hlen[g] = head ? bl[k] : 0u;
-        if (chr[k] < n_names) known[f] = 1u;  // files.rs:106-129: a consensus chromosome creates the barcode's entry
+        id[g] = f;
+        wlen[k] = head ? bl[k] : 0u;
+        if (head) klen[s] = bl[k];
+        if (known && in_table && chr[k] < n_names) known[s] = 1u;  // files.rs:106-129: a consensus chromosome creates the barcode's entry
         const unsigned m = __ballot_sync(__activemask(), head);
         if (head && (threadIdx.x & 31) == (unsigned)(__ffs(m) - 1)) atomicAdd(n_new, (uint32_t)__popc(m));
     }
 }
 
-__global__ void ingest_barcode_claim_kernel(uint32_t n, uint32_t base, const char* __restrict__ text, const uint32_t* __restrict__ slot_of,
-                                            const uint32_t* __restrict__ fidx, const uint32_t* __restrict__ bo,
-                                            const uint32_t* __restrict__ bl, const uint32_t* __restrict__ wpos, uint64_t used,
-                                            char* __restrict__ arena, unsigned long long* __restrict__ soff, uint64_t byte0,
-                                            unsigned long long* __restrict__ first_byte) {
+__global__ void ingest_key_claim_kernel(uint32_t n, uint32_t base, const char* __restrict__ text, const uint32_t* __restrict__ slot_of,
+                                        const uint32_t* __restrict__ id, const uint32_t* __restrict__ bo, const uint32_t* __restrict__ bl,
+                                        const uint32_t* __restrict__ wpos, uint64_t used, char* __restrict__ arena,
+                                        unsigned long long* __restrict__ soff, uint64_t byte0, unsigned long long* __restrict__ first_byte) {
     const uint32_t stride = gridDim.x * blockDim.x;
     for (uint32_t k = blockIdx.x * blockDim.x + threadIdx.x; k < n; k += stride) {
-        if (fidx[base + k] != base + k) continue;
+        if (id[base + k] != base + k) continue;
         const uint64_t p = used + wpos[k];
         for (uint32_t i = 0; i < bl[k]; ++i) arena[p + i] = text[bo[k] + i];
         soff[slot_of[k]] = p;
-        if (first_byte) first_byte[base + k] = byte0 + bo[k];
+        if (first_byte) first_byte[slot_of[k]] = byte0 + bo[k];
     }
 }
 
-// every later fragment of a barcode has its first appearance's bytes (a 64-bit hash collision would merge two barcodes)
-__global__ void ingest_barcode_check_kernel(uint32_t n, uint32_t base, const char* __restrict__ text, const uint32_t* __restrict__ slot_of,
-                                            const uint32_t* __restrict__ fidx, const uint32_t* __restrict__ bo,
-                                            const uint32_t* __restrict__ bl, const uint32_t* __restrict__ hlen,
-                                            const char* __restrict__ arena, const unsigned long long* __restrict__ soff,
-                                            uint32_t* __restrict__ collision) {
+// every later line of a key has its first appearance's bytes (a 64-bit hash collision would merge two keys)
+__global__ void ingest_key_check_kernel(uint32_t n, uint32_t base, const char* __restrict__ text, const uint32_t* __restrict__ slot_of,
+                                        const uint32_t* __restrict__ id, const uint32_t* __restrict__ bo, const uint32_t* __restrict__ bl,
+                                        const uint32_t* __restrict__ klen, const char* __restrict__ arena,
+                                        const unsigned long long* __restrict__ soff, uint32_t* __restrict__ collision) {
     const uint32_t stride = gridDim.x * blockDim.x;
     for (uint32_t k = blockIdx.x * blockDim.x + threadIdx.x; k < n; k += stride) {
-        const uint32_t f = fidx[base + k];
-        if (f == base + k) continue;
-        const uint64_t p = soff[slot_of[k]];
-        bool same = hlen[f] == bl[k];
+        if (id[base + k] == base + k) continue;
+        const uint32_t s = slot_of[k];
+        const uint64_t p = soff[s];
+        bool same = klen[s] == bl[k];
         for (uint32_t i = 0; same && i < bl[k]; ++i) same = arena[p + i] == text[bo[k] + i];
         if (!same) *collision = 1;
     }
 }
 
-// after the last window: a barcode is kept when keep_all is set or it was seen on a known chromosome; alen / klen are the byte
-// lengths of every first appearance / of the kept ones (u64 for the scans)
-__global__ void ingest_barcode_keep_kernel(uint64_t n, uint32_t keep_all, const uint32_t* __restrict__ fidx,
-                                           const uint32_t* __restrict__ known, const uint32_t* __restrict__ hlen,
-                                           uint32_t* __restrict__ keep, unsigned long long* __restrict__ alen,
-                                           unsigned long long* __restrict__ klen) {
+// after the last window: the first appearance and slot of every kept key (keep_all <=> known == nullptr), in no particular order
+__global__ void ingest_key_kept_kernel(uint64_t cap, const unsigned long long* __restrict__ hash, const uint32_t* __restrict__ first,
+                                       const uint32_t* __restrict__ known, uint32_t* __restrict__ kfirst, uint32_t* __restrict__ kslot,
+                                       uint32_t* __restrict__ n_kept) {
     const uint64_t stride = (uint64_t)gridDim.x * blockDim.x;
-    for (uint64_t g = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x; g < n; g += stride) {
-        const bool kp = fidx[g] == g && (keep_all || known[g]);
-        keep[g] = kp;
-        alen[g] = hlen[g];
-        klen[g] = kp ? hlen[g] : 0u;
+    for (uint64_t s = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x; s < cap; s += stride) {
+        const bool kp = hash[s] && (!known || known[s]);
+        const unsigned act = __activemask(), m = __ballot_sync(act, kp);
+        if (!m) continue;  // uniform over the active lanes
+        const int lane = threadIdx.x & 31, leader = __ffs(m) - 1;
+        uint32_t at = 0;
+        if (lane == leader) at = atomicAdd(n_kept, (uint32_t)__popc(m));
+        at = __shfl_sync(act, at, leader) + __popc(m & ((1u << lane) - 1));
+        if (kp) {
+            kfirst[at] = first[s];
+            kslot[at] = (uint32_t)s;
+        }
     }
 }
 
-// dense ids in first-appearance order among the kept barcodes; a fragment of a dropped barcode lies on an unknown chromosome
-// (it has no hit), so any valid id serves it.  The kept names are gathered from the arena in id order (blob != nullptr), or
-// their (first byte, length) spans are written in id order (spans != nullptr).
-__global__ void ingest_barcode_final_kernel(uint64_t n, const uint32_t* __restrict__ fidx, const uint32_t* __restrict__ keep,
-                                            const uint32_t* __restrict__ rank, const unsigned long long* __restrict__ aoff,
-                                            const unsigned long long* __restrict__ boff, const uint32_t* __restrict__ hlen,
-                                            const char* __restrict__ arena, char* __restrict__ blob,
-                                            unsigned long long* __restrict__ name_off, const unsigned long long* __restrict__ first_byte,
-                                            uint32_t* __restrict__ spans, uint32_t* __restrict__ bc) {
+// kept key i (first-appearance order): its name's length (for the offset scan), or its (first byte, length) span
+__global__ void ingest_key_lengths_kernel(uint32_t n_kept, const uint32_t* __restrict__ kslot, const uint32_t* __restrict__ klen,
+                                          const unsigned long long* __restrict__ first_byte, unsigned long long* __restrict__ len,
+                                          uint32_t* __restrict__ spans) {
+    const uint32_t stride = gridDim.x * blockDim.x;
+    for (uint32_t i = blockIdx.x * blockDim.x + threadIdx.x; i < n_kept; i += stride) {
+        const uint32_t s = kslot[i];
+        if (len) len[i] = klen[s];
+        if (spans) {
+            spans[2 * (uint64_t)i] = (uint32_t)first_byte[s];
+            spans[2 * (uint64_t)i + 1] = klen[s];
+        }
+    }
+}
+
+__global__ void ingest_key_names_kernel(uint32_t n_kept, const uint32_t* __restrict__ kslot, const uint32_t* __restrict__ klen,
+                                        const unsigned long long* __restrict__ soff, const char* __restrict__ arena,
+                                        const unsigned long long* __restrict__ name_off, char* __restrict__ blob) {
+    const uint32_t stride = gridDim.x * blockDim.x;
+    for (uint32_t i = blockIdx.x * blockDim.x + threadIdx.x; i < n_kept; i += stride) {
+        const uint32_t s = kslot[i];
+        for (uint32_t j = 0; j < klen[s]; ++j) blob[name_off[i] + j] = arena[soff[s] + j];
+    }
+}
+
+// a line's first-appearance index -> its key's dense id: the index's position among the kept keys' sorted first appearances.
+// A line of a dropped key lies on an unknown chromosome (it has no hit), so any valid id serves it.
+__global__ void ingest_key_ids_kernel(uint64_t n, const uint32_t* __restrict__ kfirst, uint32_t n_kept, uint32_t* __restrict__ id) {
     const uint64_t stride = (uint64_t)gridDim.x * blockDim.x;
     for (uint64_t g = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x; g < n; g += stride) {
-        const uint32_t f = fidx[g];
-        bc[g] = keep[f] ? rank[f] : 0u;
-        if (keep[g]) {
-            if (blob) {
-                for (uint32_t i = 0; i < hlen[g]; ++i) blob[boff[g] + i] = arena[aoff[g] + i];
-                name_off[rank[g]] = boff[g];
-            }
-            if (spans) {
-                spans[2 * (uint64_t)rank[g]] = (uint32_t)first_byte[g];
-                spans[2 * (uint64_t)rank[g] + 1] = hlen[g];
-            }
-        }
+        const uint32_t f = id[g], i = lower_bound_u32(kfirst, n_kept, f);
+        id[g] = i < n_kept && kfirst[i] == f ? i : 0u;
     }
 }
 
@@ -466,35 +458,43 @@ static int igrid(gtgpu_ctx* ctx, uint64_t n) {
     return (int)std::max<uint64_t>(1, std::min<uint64_t>((n + 255) / 256, (uint64_t)ctx->sm_count * 16));
 }
 
-// Fragment name table in scratch SC_SET_ID: FNV-1a hashes of the caller's chromosome names, sorted for the device lookup.
-int32_t upload_name_table(gtgpu_ctx* ctx, uint32_t n_names, const char* names, const uint32_t* name_offsets, NameTable* out) {
+// Name table in scratch SC_SET_ID: FNV-1a hashes of the caller's chromosome names, sorted for the device lookup, and (with_rank)
+// the names' lexicographic ranks for the sort of gtgpu_parse_bed.
+int32_t upload_name_table(gtgpu_ctx* ctx, uint32_t n_names, const char* names, const uint32_t* name_offsets, NameTable* out,
+                          bool with_rank) {
     cudaStream_t st = ctx->stream;
     std::vector<unsigned long long> hash(n_names), hash_sorted(n_names);
-    std::vector<uint32_t> hash_id(n_names);
-    for (uint32_t i = 0; i < n_names; ++i) {
-        unsigned long long h = 1469598103934665603ull;
-        for (uint32_t k = name_offsets[i]; k < name_offsets[i + 1]; ++k) h = (h ^ (unsigned char)names[k]) * 1099511628211ull;
-        hash[i] = h;
-    }
+    std::vector<uint32_t> hash_id(n_names), rank(with_rank ? n_names : 0);
+    for (uint32_t i = 0; i < n_names; ++i) hash[i] = fnv1a64(names + name_offsets[i], name_offsets[i + 1] - name_offsets[i]);
     std::iota(hash_id.begin(), hash_id.end(), 0u);
     std::sort(hash_id.begin(), hash_id.end(), [&](uint32_t a, uint32_t b) { return hash[a] != hash[b] ? hash[a] < hash[b] : a < b; });
     for (uint32_t i = 0; i < n_names; ++i) hash_sorted[i] = hash[hash_id[i]];
+    if (with_rank) {
+        std::vector<uint32_t> by_name(n_names);
+        std::iota(by_name.begin(), by_name.end(), 0u);
+        auto name_of = [&](uint32_t i) { return std::string(names + name_offsets[i], names + name_offsets[i + 1]); };
+        std::stable_sort(by_name.begin(), by_name.end(), [&](uint32_t a, uint32_t b) { return name_of(a) < name_of(b); });
+        for (uint32_t r = 0; r < n_names; ++r) rank[by_name[r]] = r;  // equal strings cannot occur in a name table
+    }
     const uint32_t blob_bytes = n_names ? name_offsets[n_names] : 0;
     char* d_names;
     GT_TRY(ctx->scratch_get(SC_SET_ID, (size_t)n_names * 16 + ((size_t)n_names + 1) * 4 + blob_bytes + 64, (void**)&d_names));
+    // layout: hashes (8-byte aligned first), offsets, hash ids, ranks, blob
     unsigned long long* d_hash = reinterpret_cast<unsigned long long*>(d_names);
     uint32_t* d_noff = reinterpret_cast<uint32_t*>(d_hash + n_names);
     uint32_t* d_hid = d_noff + n_names + 1;
-    char* d_blob = reinterpret_cast<char*>(d_hid + n_names);
+    uint32_t* d_rank = d_hid + n_names;
+    char* d_blob = reinterpret_cast<char*>(d_rank + n_names);
     if (n_names) {
         GT_CUDA(cudaMemcpyAsync(d_hash, hash_sorted.data(), (size_t)n_names * 8, cudaMemcpyHostToDevice, st));
         GT_CUDA(cudaMemcpyAsync(d_hid, hash_id.data(), (size_t)n_names * 4, cudaMemcpyHostToDevice, st));
+        if (with_rank) GT_CUDA(cudaMemcpyAsync(d_rank, rank.data(), (size_t)n_names * 4, cudaMemcpyHostToDevice, st));
         if (blob_bytes) GT_CUDA(cudaMemcpyAsync(d_blob, names, blob_bytes, cudaMemcpyHostToDevice, st));
     }
     GT_CUDA(cudaMemcpyAsync(d_noff, name_offsets ? name_offsets : (const uint32_t*)&blob_bytes, ((size_t)n_names + 1) * 4,
                             cudaMemcpyHostToDevice, st));
     GT_CUDA(cudaStreamSynchronize(st));  // the host vectors above are pageable and go out of scope
-    *out = NameTable{d_blob, d_noff, d_hash, d_hid, n_names};
+    *out = NameTable{d_blob, d_noff, d_hash, d_hid, n_names, with_rank ? d_rank : nullptr};
     return GTGPU_OK;
 }
 
@@ -526,70 +526,79 @@ static int32_t line_breaks_locked(gtgpu_ctx* ctx, const char* d_text, uint64_t n
     return GTGPU_OK;
 }
 
-// The fragment front end shared by tokenize_fragment_file and the scoring entry points: newline positions, one thread per
-// line, compaction of the kept lines.  d_text: 0 < n_bytes < 0xFFFFFFF0 bytes of device text, 16-byte aligned.
-int32_t parse_fragments_locked(gtgpu_ctx* ctx, const char* d_text, uint64_t n_bytes, const NameTable& nt, FragMode mode,
-                               FragParse* out) {
+// The line front end of every device text parser: line breaks, the format's line kernel, compaction of the kept lines.
+int32_t parse_lines_locked(gtgpu_ctx* ctx, const char* d_text, uint64_t n_bytes, LineFormat fmt, const NameTable& nt,
+                           const BedFilesView& files, ParsedLines* out) {
     cudaStream_t st = ctx->stream;
-    uint32_t* d_nl;
+    uint32_t *d_nl, *d_pos;
     void* d_tmp;
-    uint32_t n_newlines, n_lines;
-    GT_TRY(line_breaks_locked(ctx, d_text, n_bytes, nullptr, 0, &n_newlines, &n_lines, &d_nl));
-    // ---- parse + compact ---------------------------------------------------------------------------------------------------
-    const bool bc = mode != FRAG_SCORE_MATRIX;
-    const size_t lb = (size_t)n_lines * 4 + 8;
-    uint32_t *d_keep, *d_pos, *p_chr, *p_start, *p_end, *p_bo = nullptr, *p_bl = nullptr, *o_chr, *o_start, *o_end, *o_bo = nullptr,
-             *o_bl = nullptr;
-    unsigned long long *p_h = nullptr, *o_h = nullptr;
     uint64_t* d_misc;
+    uint32_t n_breaks = 0, n_lines = 0;
+    GT_TRY(line_breaks_locked(ctx, d_text, n_bytes, files.fstart, files.n_fstart, &n_breaks, &n_lines, &d_nl));
+    const bool keys = fmt == BED_FILE_LINES || fmt == FRAG_TOKENIZE || fmt == FRAG_SCORE_BARCODES;
+    const size_t lb = (size_t)n_lines * 4 + 8;
+    LineCols p{}, o{};  // per line, per kept line
     GT_TRY(ctx->scratch_get(SC_IN3_START, exclusive_scan_temp_bytes(n_lines, 4), &d_tmp));
-    GT_TRY(ctx->scratch_get(SC_ING_0, lb, (void**)&d_keep));
+    GT_TRY(ctx->scratch_get(SC_ING_0, lb, (void**)&p.keep));
     GT_TRY(ctx->scratch_get(SC_ING_1, lb, (void**)&d_pos));
-    GT_TRY(ctx->scratch_get(SC_IN2_CHR, lb, (void**)&p_chr));
-    GT_TRY(ctx->scratch_get(SC_IN2_START, lb, (void**)&p_start));
-    GT_TRY(ctx->scratch_get(SC_IN2_END, lb, (void**)&p_end));
-    GT_TRY(ctx->scratch_get(SC_CHR, lb, (void**)&o_chr));
-    GT_TRY(ctx->scratch_get(SC_START, lb, (void**)&o_start));
-    GT_TRY(ctx->scratch_get(SC_END, lb, (void**)&o_end));
-    if (bc) {
-        GT_TRY(ctx->scratch_get(SC_ING_2, lb * 2, (void**)&p_h));
-        GT_TRY(ctx->scratch_get(SC_ING_3, lb, (void**)&p_bo));
-        GT_TRY(ctx->scratch_get(SC_ING_4, lb, (void**)&p_bl));
-        GT_TRY(ctx->scratch_get(SC_ING_5, lb * 2, (void**)&o_h));
-        GT_TRY(ctx->scratch_get(SC_ING_6, lb, (void**)&o_bo));
-        GT_TRY(ctx->scratch_get(SC_ING_7, lb, (void**)&o_bl));
+    GT_TRY(ctx->scratch_get(SC_IN2_CHR, lb, (void**)&p.chr));
+    GT_TRY(ctx->scratch_get(SC_IN2_START, lb, (void**)&p.start));
+    GT_TRY(ctx->scratch_get(SC_IN2_END, lb, (void**)&p.end));
+    GT_TRY(ctx->scratch_get(SC_CHR, lb, (void**)&o.chr));
+    GT_TRY(ctx->scratch_get(SC_START, lb, (void**)&o.start));
+    GT_TRY(ctx->scratch_get(SC_END, lb, (void**)&o.end));
+    if (keys) {
+        GT_TRY(ctx->scratch_get(SC_ING_2, lb * 2, (void**)&p.h));
+        GT_TRY(ctx->scratch_get(SC_ING_3, lb, (void**)&p.bo));
+        GT_TRY(ctx->scratch_get(SC_ING_4, lb, (void**)&p.bl));
+        GT_TRY(ctx->scratch_get(SC_ING_5, lb * 2, (void**)&o.h));
+        GT_TRY(ctx->scratch_get(SC_ING_6, lb, (void**)&o.bo));
+        GT_TRY(ctx->scratch_get(SC_ING_7, lb, (void**)&o.bl));
     }
     GT_TRY(ctx->scratch_get(SC_MISC, 64, (void**)&d_misc));
-    uint32_t* d_flags = reinterpret_cast<uint32_t*>(d_misc);  // [0] first malformed line, [1..3] for the caller's barcode table
+    uint32_t* d_flags = reinterpret_cast<uint32_t*>(d_misc);  // [0] first malformed line, [1..3] for the caller
     const uint32_t init[4] = {0xFFFFFFFFu, 0u, 0u, 0u};
     GT_CUDA(cudaMemcpyAsync(d_flags, init, 16, cudaMemcpyHostToDevice, st));
-    auto kern = mode == FRAG_TOKENIZE ? ingest_parse_fragments_kernel<false, true>
-                : mode == FRAG_SCORE_MATRIX ? ingest_parse_fragments_kernel<true, false> : ingest_parse_fragments_kernel<true, true>;
-    kern<<<igrid(ctx, n_lines), 256, 0, st>>>(n_lines, n_newlines, n_bytes, d_text, d_nl, nt, d_keep, p_chr, p_start, p_end, p_h, p_bo,
-                                              p_bl, d_flags);
+    const int grid = igrid(ctx, n_lines);
+    switch (fmt) {
+    case BED_LINES:
+        ingest_parse_lines_kernel<false><<<grid, 256, 0, st>>>(n_lines, n_breaks, n_bytes, d_text, d_nl, nt, p, d_flags, files);
+        break;
+    case BED_FILE_LINES:
+        ingest_parse_lines_kernel<true><<<grid, 256, 0, st>>>(n_lines, n_breaks, n_bytes, d_text, d_nl, nt, p, d_flags, files);
+        break;
+    case FRAG_TOKENIZE:
+        ingest_parse_fragments_kernel<false, true><<<grid, 256, 0, st>>>(n_lines, n_breaks, n_bytes, d_text, d_nl, nt, p, d_flags);
+        break;
+    case FRAG_SCORE_MATRIX:
+        ingest_parse_fragments_kernel<true, false><<<grid, 256, 0, st>>>(n_lines, n_breaks, n_bytes, d_text, d_nl, nt, p, d_flags);
+        break;
+    case FRAG_SCORE_BARCODES:
+        ingest_parse_fragments_kernel<true, true><<<grid, 256, 0, st>>>(n_lines, n_breaks, n_bytes, d_text, d_nl, nt, p, d_flags);
+        break;
+    }
     ctx->launches++;
-    GT_TRY(exclusive_scan<uint32_t>(ctx, d_keep, d_pos, n_lines, d_tmp));
-    ingest_compact_fragments_kernel<<<igrid(ctx, n_lines), 256, 0, st>>>(n_lines, d_keep, d_pos, p_chr, p_start, p_end, p_h, p_bo, p_bl,
-                                                                         o_chr, o_start, o_end, o_h, o_bo, o_bl);
+    GT_TRY(exclusive_scan<uint32_t>(ctx, p.keep, d_pos, n_lines, d_tmp));
+    ingest_compact_lines_kernel<<<grid, 256, 0, st>>>(n_lines, d_pos, p, o);
     ctx->launches++;
     uint32_t tail[2], flags[1];
     GT_CUDA(cudaMemcpyAsync(&tail[0], d_pos + n_lines - 1, 4, cudaMemcpyDeviceToHost, st));
-    GT_CUDA(cudaMemcpyAsync(&tail[1], d_keep + n_lines - 1, 4, cudaMemcpyDeviceToHost, st));
+    GT_CUDA(cudaMemcpyAsync(&tail[1], p.keep + n_lines - 1, 4, cudaMemcpyDeviceToHost, st));
     GT_CUDA(cudaMemcpyAsync(flags, d_flags, 4, cudaMemcpyDeviceToHost, st));
     GT_CUDA(cudaStreamSynchronize(st));
-    *out = FragParse{};
+    *out = ParsedLines{};
     out->n_lines = n_lines;
     out->bad_line = flags[0];
     out->n = flags[0] == 0xFFFFFFFFu ? tail[0] + tail[1] : 0;
-    out->chr = o_chr;
-    out->start = o_start;
-    out->end = o_end;
-    out->h = o_h;
-    out->bo = o_bo;
-    out->bl = o_bl;
-    out->free0 = d_keep;  // the line-sized arrays are free again
-    out->free1 = d_pos;
-    out->free2 = p_chr;
+    out->chr = o.chr;
+    out->start = o.start;
+    out->end = o.end;
+    out->h = o.h;
+    out->bo = o.bo;
+    out->bl = o.bl;
+    out->breaks = d_nl;
+    uint32_t* const line_sized[5] = {p.keep, d_pos, p.chr, p.start, p.end};  // free again
+    std::copy(line_sized, line_sized + 5, out->free);
     out->tmp = d_tmp;
     out->flags = d_flags;
     return GTGPU_OK;
@@ -726,109 +735,31 @@ static int32_t parse_bed_locked(gtgpu_ctx* ctx, const char* host_text, const cha
     *n_out = 0;
     if (n_bytes == 0) return fail(GTGPU_ERR_INVALID, "parse_bed: EmptyRegionSet (no regions in the text)");
 
-    // ---- name table: hashes sorted for the device lookup, lexicographic ranks for the sort ----------------------------
-    std::vector<unsigned long long> hash(n_names);
-    std::vector<uint32_t> hash_id(n_names), rank(n_names), by_name(n_names);
-    for (uint32_t i = 0; i < n_names; ++i) {
-        unsigned long long h = 1469598103934665603ull;
-        for (uint32_t k = name_offsets[i]; k < name_offsets[i + 1]; ++k) h = (h ^ (unsigned char)names[k]) * 1099511628211ull;
-        hash[i] = h;
-    }
-    std::iota(hash_id.begin(), hash_id.end(), 0u);
-    std::sort(hash_id.begin(), hash_id.end(), [&](uint32_t a, uint32_t b) { return hash[a] != hash[b] ? hash[a] < hash[b] : a < b; });
-    std::vector<unsigned long long> hash_sorted(n_names);
-    for (uint32_t i = 0; i < n_names; ++i) hash_sorted[i] = hash[hash_id[i]];
-    std::iota(by_name.begin(), by_name.end(), 0u);
-    auto name_of = [&](uint32_t i) { return std::string(names + name_offsets[i], names + name_offsets[i + 1]); };
-    std::stable_sort(by_name.begin(), by_name.end(), [&](uint32_t a, uint32_t b) { return name_of(a) < name_of(b); });
-    for (uint32_t r = 0; r < n_names; ++r) rank[by_name[r]] = r;  // equal strings cannot occur in a name table
-    const uint32_t blob_bytes = n_names ? name_offsets[n_names] : 0;
-
     const char* d_text = dev_text;
-    uint32_t *d_counts, *d_crank, *d_nl;
-    void* d_tmp;
-    char* d_names;
-    const uint64_t n_chunks = (n_bytes + INGEST_CHUNK - 1) / INGEST_CHUNK;
-    if (!dev_text) GT_TRY(ctx->scratch_get(SC_OUT_IDS2, n_bytes + 64, (void**)&d_text));
-    GT_TRY(ctx->scratch_get(SC_COUNTS, n_chunks * 4 + 4, (void**)&d_counts));
-    GT_TRY(ctx->scratch_get(SC_IN3_CHR, n_chunks * 4 + 4, (void**)&d_crank));
-    const size_t names_bytes = ((size_t)blob_bytes + 15) / 16 * 16 + ((size_t)n_names + 1) * 4 + (size_t)n_names * 8 + (size_t)n_names * 4 * 2 + 64;
-    GT_TRY(ctx->scratch_get(SC_SET_ID, names_bytes, (void**)&d_names));
-    if (!dev_text) GT_CUDA(cudaMemcpyAsync((char*)d_text, host_text, n_bytes, cudaMemcpyHostToDevice, st));
-    // layout of the name scratch: hashes (8-byte aligned first), offsets, hash ids, ranks, blob
-    unsigned long long* d_hash = reinterpret_cast<unsigned long long*>(d_names);
-    uint32_t* d_noff = reinterpret_cast<uint32_t*>(d_hash + n_names);
-    uint32_t* d_hid = d_noff + n_names + 1;
-    uint32_t* d_rank = d_hid + n_names;
-    char* d_blob = reinterpret_cast<char*>(d_rank + n_names);
-    if (n_names) {
-        GT_CUDA(cudaMemcpyAsync(d_hash, hash_sorted.data(), (size_t)n_names * 8, cudaMemcpyHostToDevice, st));
-        GT_CUDA(cudaMemcpyAsync(d_hid, hash_id.data(), (size_t)n_names * 4, cudaMemcpyHostToDevice, st));
-        GT_CUDA(cudaMemcpyAsync(d_rank, rank.data(), (size_t)n_names * 4, cudaMemcpyHostToDevice, st));
-        if (blob_bytes) GT_CUDA(cudaMemcpyAsync(d_blob, names, blob_bytes, cudaMemcpyHostToDevice, st));
+    if (!dev_text) {
+        GT_TRY(ctx->scratch_get(SC_OUT_IDS2, n_bytes + 64, (void**)&d_text));
+        GT_CUDA(cudaMemcpyAsync((char*)d_text, host_text, n_bytes, cudaMemcpyHostToDevice, st));
     }
-    GT_CUDA(cudaMemcpyAsync(d_noff, name_offsets ? name_offsets : (const uint32_t*)&blob_bytes, ((size_t)n_names + 1) * 4,
-                            cudaMemcpyHostToDevice, st));
-
-    // ---- 1. newline positions ---------------------------------------------------------------------------------------------
-    GT_TRY(ctx->scratch_get(SC_IN3_START, exclusive_scan_temp_bytes(n_chunks, 4), &d_tmp));
-    ingest_count_newlines_kernel<<<igrid(ctx, n_chunks), 256, 0, st>>>(n_bytes, d_text, d_counts, nullptr, 0);
-    ctx->launches++;
-    GT_TRY(exclusive_scan<uint32_t>(ctx, d_counts, d_crank, n_chunks, d_tmp));
-    uint32_t last[2];
-    GT_CUDA(cudaMemcpyAsync(&last[0], d_crank + n_chunks - 1, 4, cudaMemcpyDeviceToHost, st));
-    GT_CUDA(cudaMemcpyAsync(&last[1], d_counts + n_chunks - 1, 4, cudaMemcpyDeviceToHost, st));
-    char last_byte = 0;  // read back from the device: with device-resident text there is no host copy
-    GT_CUDA(cudaMemcpyAsync(&last_byte, d_text + n_bytes - 1, 1, cudaMemcpyDeviceToHost, st));
-    GT_CUDA(cudaStreamSynchronize(st));  // the host's text buffer may be reused after this point
-    const uint32_t n_newlines = last[0] + last[1];
-    const uint32_t n_lines = n_newlines + (last_byte != '\n' ? 1u : 0u);
-    GT_TRY(ctx->scratch_get(SC_IN3_END, (size_t)n_newlines * 4 + 4, (void**)&d_nl));
-    ingest_newline_positions_kernel<<<igrid(ctx, n_chunks), 256, 0, st>>>(n_bytes, d_text, d_crank, d_nl, nullptr, 0);
-    ctx->launches++;
-
-    // ---- 2. parse, 3. compact ---------------------------------------------------------------------------------------------
-    uint32_t *d_keep, *d_pos, *p_chr, *p_start, *p_end, *o_chr, *o_start, *o_end;
-    uint64_t* d_misc;
-    const size_t lb = (size_t)n_lines * 4 + 4;
-    GT_TRY(ctx->scratch_get(SC_IN3_START, std::max(exclusive_scan_temp_bytes(n_lines, 4), radix_sort_temp_bytes(n_lines)), &d_tmp));
-    GT_TRY(ctx->scratch_get(SC_BARCODE, lb, (void**)&d_keep));
-    GT_TRY(ctx->scratch_get(SC_FILE_TOK2, lb, (void**)&d_pos));
-    GT_TRY(ctx->scratch_get(SC_IN2_CHR, lb, (void**)&p_chr));
-    GT_TRY(ctx->scratch_get(SC_IN2_START, lb, (void**)&p_start));
-    GT_TRY(ctx->scratch_get(SC_IN2_END, lb, (void**)&p_end));
-    GT_TRY(ctx->scratch_get(SC_CHR, lb, (void**)&o_chr));
-    GT_TRY(ctx->scratch_get(SC_START, lb, (void**)&o_start));
-    GT_TRY(ctx->scratch_get(SC_END, lb, (void**)&o_end));
-    GT_TRY(ctx->scratch_get(SC_MISC, 64, (void**)&d_misc));
-    uint32_t* d_flags = reinterpret_cast<uint32_t*>(d_misc);  // [0] first malformed line, [1] unsorted
-    const uint32_t init[2] = {0xFFFFFFFFu, 0u};
-    GT_CUDA(cudaMemcpyAsync(d_flags, init, 8, cudaMemcpyHostToDevice, st));
-    NameTable nt{d_blob, d_noff, d_hash, d_hid, n_names};
-    ingest_parse_lines_kernel<false><<<igrid(ctx, n_lines), 256, 0, st>>>(n_lines, n_newlines, n_bytes, d_text, d_nl, nt, d_keep, p_chr,
-                                                                          p_start, p_end, d_flags, BedFilesView{});
-    ctx->launches++;
-    GT_TRY(exclusive_scan<uint32_t>(ctx, d_keep, d_pos, n_lines, d_tmp));
-    ingest_compact_kernel<<<igrid(ctx, n_lines), 256, 0, st>>>(n_lines, d_keep, d_pos, p_chr, p_start, p_end, o_chr, o_start, o_end);
-    ctx->launches++;
-    uint32_t tail[2], flags[2];
-    GT_CUDA(cudaMemcpyAsync(&tail[0], d_pos + n_lines - 1, 4, cudaMemcpyDeviceToHost, st));
-    GT_CUDA(cudaMemcpyAsync(&tail[1], d_keep + n_lines - 1, 4, cudaMemcpyDeviceToHost, st));
-    GT_CUDA(cudaMemcpyAsync(flags, d_flags, 4, cudaMemcpyDeviceToHost, st));
-    GT_CUDA(cudaStreamSynchronize(st));
-    if (flags[0] != 0xFFFFFFFFu)
-        return fail(GTGPU_ERR_INVALID, "parse_bed: RegionParseError: cannot parse start / end position on line " + std::to_string((uint64_t)flags[0] + 1));
-    const uint32_t n = tail[0] + tail[1];
+    NameTable nt;
+    GT_TRY(upload_name_table(ctx, n_names, names, name_offsets, &nt, true));  // synchronises: the host's text may be reused after it
+    ParsedLines pl;
+    GT_TRY(parse_lines_locked(ctx, d_text, n_bytes, BED_LINES, nt, BedFilesView{}, &pl));
+    if (pl.bad_line != 0xFFFFFFFFu)
+        return fail(GTGPU_ERR_INVALID, "parse_bed: RegionParseError: cannot parse start / end position on line " + std::to_string((uint64_t)pl.bad_line + 1));
+    const uint32_t n = pl.n;
     if (n == 0) return fail(GTGPU_ERR_INVALID, "parse_bed: EmptyRegionSet (no regions in the text)");
+    uint32_t *o_chr = pl.chr, *o_start = pl.start, *o_end = pl.end, *d_flags = pl.flags, flags[2];
 
     // ---- 4. RegionSet::sort: stable by (chromosome string, start) -----------------------------------------------------------
-    ingest_check_sorted_kernel<<<igrid(ctx, n), 256, 0, st>>>(n, o_chr, o_start, d_rank, n_names, d_flags + 1);
+    ingest_check_sorted_kernel<<<igrid(ctx, n), 256, 0, st>>>(n, o_chr, o_start, nt.rank, n_names, d_flags + 1);
     ctx->launches++;
     GT_CUDA(cudaMemcpyAsync(flags, d_flags, 8, cudaMemcpyDeviceToHost, st));
     GT_CUDA(cudaStreamSynchronize(st));
     if (flags[1]) {
-        uint32_t *k_a = d_keep, *v_a = d_pos, *k_b, *v_b;  // the line-sized arrays are free again
+        uint32_t *k_a = pl.free[0], *v_a = pl.free[1], *k_b, *v_b, *g_chr = pl.free[2], *g_start = pl.free[3], *g_end = pl.free[4];
+        void* d_tmp;
         GT_TRY(ctx->scratch_get(SC_OUT_IDS, (size_t)n * 8 + 8, (void**)&k_b));
+        GT_TRY(ctx->scratch_get(SC_IN3_START, radix_sort_temp_bytes(n), &d_tmp));
         v_b = k_b + n;
         GT_CUDA(cudaMemcpyAsync(k_a, o_start, (size_t)n * 4, cudaMemcpyDeviceToDevice, st));
         ingest_iota_kernel<<<igrid(ctx, n), 256, 0, st>>>(n, v_a);
@@ -836,15 +767,15 @@ static int32_t parse_bed_locked(gtgpu_ctx* ctx, const char* host_text, const cha
         int in_b = 0;
         GT_TRY(radix_sort_pairs(ctx, n, k_a, v_a, k_b, v_b, 32, d_tmp, &in_b));
         if (in_b) { std::swap(k_a, k_b); std::swap(v_a, v_b); }
-        ingest_rank_keys_kernel<<<igrid(ctx, n), 256, 0, st>>>(n, v_a, o_chr, d_rank, n_names, k_a);
+        ingest_rank_keys_kernel<<<igrid(ctx, n), 256, 0, st>>>(n, v_a, o_chr, nt.rank, n_names, k_a);
         ctx->launches++;
         int bits = 1;
         while (bits < 32 && (1ull << bits) < (uint64_t)n_names + 1) ++bits;
         GT_TRY(radix_sort_pairs(ctx, n, k_a, v_a, k_b, v_b, bits, d_tmp, &in_b));
         const uint32_t* order = in_b ? v_b : v_a;
-        ingest_gather_kernel<<<igrid(ctx, n), 256, 0, st>>>(n, order, o_chr, o_start, o_end, p_chr, p_start, p_end);
+        ingest_gather_kernel<<<igrid(ctx, n), 256, 0, st>>>(n, order, o_chr, o_start, o_end, g_chr, g_start, g_end);
         ctx->launches++;
-        o_chr = p_chr; o_start = p_start; o_end = p_end;
+        o_chr = g_chr; o_start = g_start; o_end = g_end;
     }
     GT_CUDA(cudaGetLastError());
     *n_out = n;
@@ -876,133 +807,157 @@ DevMem::~DevMem() {
     if (ptr) cudaFree(ptr);
 }
 
-int32_t FragBarcodeTable::add_window(gtgpu_ctx* ctx, const char* d_text, uint64_t byte0, const FragParse& fp, uint32_t n_names) {
-    const uint32_t nw = fp.n;
+static KeySlots key_slots(DevMem& hash, DevMem& soff, DevMem& first_byte, DevMem& first, DevMem& klen, DevMem& known) {
+    return KeySlots{(unsigned long long*)hash.ptr, (unsigned long long*)soff.ptr, (unsigned long long*)first_byte.ptr,
+                    first.u32(), klen.u32(), known.u32()};
+}
+
+int32_t KeyTable::add_window(gtgpu_ctx* ctx, const char* d_text, uint64_t byte0, const ParsedLines& pl, uint32_t n_names) {
+    const uint32_t nw = pl.n;
     if (nw == 0) return GTGPU_OK;
     cudaStream_t st = ctx->stream;
     const uint32_t base = (uint32_t)n;
     const size_t need = (size_t)(n + nw) * 4, have = (size_t)n * 4;
-    for (DevMem* m : {&chr, &start, &end, &fidx, &known, &hlen}) GT_TRY(m->reserve(need, have, st));
-    if (record_spans) GT_TRY(first_byte.reserve(need * 2, have * 2, st));
-    GT_CUDA(cudaMemcpyAsync(chr.u32() + base, fp.chr, (size_t)nw * 4, cudaMemcpyDeviceToDevice, st));
-    GT_CUDA(cudaMemcpyAsync(start.u32() + base, fp.start, (size_t)nw * 4, cudaMemcpyDeviceToDevice, st));
-    GT_CUDA(cudaMemcpyAsync(end.u32() + base, fp.end, (size_t)nw * 4, cudaMemcpyDeviceToDevice, st));
-    GT_CUDA(cudaMemsetAsync(known.u32() + base, 0, (size_t)nw * 4, st));
-    // the table holds at most distinct + nw barcodes after this window: keep it at most half full
+    for (DevMem* m : {&chr, &start, &end, &id}) GT_TRY(m->reserve(need, have, st));
+    GT_CUDA(cudaMemcpyAsync(chr.u32() + base, pl.chr, (size_t)nw * 4, cudaMemcpyDeviceToDevice, st));
+    GT_CUDA(cudaMemcpyAsync(start.u32() + base, pl.start, (size_t)nw * 4, cudaMemcpyDeviceToDevice, st));
+    GT_CUDA(cudaMemcpyAsync(end.u32() + base, pl.end, (size_t)nw * 4, cudaMemcpyDeviceToDevice, st));
+    // the table holds at most min(distinct + nw, max_keys) keys after this window (more are an error): keep it at most half full
     uint64_t new_cap = std::max<uint64_t>(cap, 1024);
-    while (new_cap < 2 * (distinct + nw)) new_cap <<= 1;
+    while (new_cap < 2 * std::min<uint64_t>(distinct + nw, max_keys)) new_cap <<= 1;
     if (new_cap != cap) {
-        DevMem k2, f2, s2;
-        GT_TRY(k2.reserve(new_cap * 8, 0, st));
-        GT_TRY(f2.reserve(new_cap * 4, 0, st));
-        GT_TRY(s2.reserve(new_cap * 8, 0, st));
-        GT_CUDA(cudaMemsetAsync(k2.ptr, 0, new_cap * 8, st));
-        GT_CUDA(cudaMemsetAsync(f2.ptr, 0xFF, new_cap * 4, st));
+        DevMem t_hash, t_soff, t_first_byte, t_first, t_klen, t_known;
+        GT_TRY(t_hash.reserve(new_cap * 8, 0, st));
+        GT_TRY(t_soff.reserve(new_cap * 8, 0, st));
+        GT_TRY(t_first.reserve(new_cap * 4, 0, st));
+        GT_TRY(t_klen.reserve(new_cap * 4, 0, st));
+        if (record_spans) GT_TRY(t_first_byte.reserve(new_cap * 8, 0, st));
+        if (!keep_all) {
+            GT_TRY(t_known.reserve(new_cap * 4, 0, st));
+            GT_CUDA(cudaMemsetAsync(t_known.ptr, 0, new_cap * 4, st));
+        }
+        GT_CUDA(cudaMemsetAsync(t_hash.ptr, 0, new_cap * 8, st));
+        GT_CUDA(cudaMemsetAsync(t_first.ptr, 0xFF, new_cap * 4, st));
         if (cap) {
-            ingest_barcode_rehash_kernel<<<igrid(ctx, cap), 256, 0, st>>>(cap, (const unsigned long long*)keys.ptr, first.u32(),
-                                                                         (const unsigned long long*)soff.ptr, (uint32_t)(new_cap - 1),
-                                                                         (unsigned long long*)k2.ptr, f2.u32(), (unsigned long long*)s2.ptr);
+            ingest_key_rehash_kernel<<<igrid(ctx, cap), 256, 0, st>>>(cap, key_slots(hash, soff, first_byte, first, klen, known),
+                                                                     (uint32_t)(new_cap - 1),
+                                                                     key_slots(t_hash, t_soff, t_first_byte, t_first, t_klen, t_known));
             ctx->launches++;
         }
         GT_CUDA(cudaStreamSynchronize(st));
-        keys.swap(k2);
-        first.swap(f2);
-        soff.swap(s2);
+        hash.swap(t_hash);
+        soff.swap(t_soff);
+        first_byte.swap(t_first_byte);
+        first.swap(t_first);
+        klen.swap(t_klen);
+        known.swap(t_known);
         cap = new_cap;
     }
-    uint32_t* slot_of = fp.free0;
-    uint32_t* wpos = fp.free1;
-    ingest_barcode_insert_kernel<<<igrid(ctx, nw), 256, 0, st>>>(nw, fp.h, (uint32_t)(cap - 1), (unsigned long long*)keys.ptr, first.u32(),
-                                                                 slot_of, base);
-    ingest_barcode_window_heads_kernel<<<igrid(ctx, nw), 256, 0, st>>>(nw, base, slot_of, first.u32(), fp.chr, fp.bl, n_names, fidx.u32(),
-                                                                       hlen.u32(), known.u32(), fp.flags + 2);
+    const uint32_t mask = (uint32_t)(cap - 1);
+    uint32_t *slot_of = pl.free[0], *wpos = pl.free[1], *wlen = pl.free[2];
+    ingest_key_insert_kernel<<<igrid(ctx, nw), 256, 0, st>>>(nw, pl.h, mask, (unsigned long long*)hash.ptr, first.u32(), slot_of, base,
+                                                             pl.flags + 3);
+    ingest_key_heads_kernel<<<igrid(ctx, nw), 256, 0, st>>>(nw, base, slot_of, first.u32(), pl.chr, pl.bl, n_names, mask, id.u32(),
+                                                            klen.u32(), known.u32(), wlen, pl.flags + 2);
     ctx->launches += 2;
-    GT_TRY(exclusive_scan<uint32_t>(ctx, hlen.u32() + base, wpos, nw, fp.tmp));
-    uint32_t tail[3];
+    GT_TRY(exclusive_scan<uint32_t>(ctx, wlen, wpos, nw, pl.tmp));
+    uint32_t tail[4];  // last offset, last length, keys first seen here, table full
     GT_CUDA(cudaMemcpyAsync(&tail[0], wpos + nw - 1, 4, cudaMemcpyDeviceToHost, st));
-    GT_CUDA(cudaMemcpyAsync(&tail[1], hlen.u32() + base + nw - 1, 4, cudaMemcpyDeviceToHost, st));
-    GT_CUDA(cudaMemcpyAsync(&tail[2], fp.flags + 2, 4, cudaMemcpyDeviceToHost, st));
+    GT_CUDA(cudaMemcpyAsync(&tail[1], wlen + nw - 1, 4, cudaMemcpyDeviceToHost, st));
+    GT_CUDA(cudaMemcpyAsync(&tail[2], pl.flags + 2, 8, cudaMemcpyDeviceToHost, st));
     GT_CUDA(cudaStreamSynchronize(st));
+    if (tail[3] || distinct + tail[2] > max_keys)
+        return fail(GTGPU_ERR_UNSUPPORTED, who + ": more than " + std::to_string(max_keys) + " distinct " + keys);
     const uint64_t bytes = (uint64_t)tail[0] + tail[1];
     GT_TRY(arena.reserve(used + bytes + 1, used, st));
-    ingest_barcode_claim_kernel<<<igrid(ctx, nw), 256, 0, st>>>(nw, base, d_text, slot_of, fidx.u32(), fp.bo, fp.bl, wpos, used,
-                                                                (char*)arena.ptr, (unsigned long long*)soff.ptr, byte0,
-                                                                (unsigned long long*)first_byte.ptr);
-    ingest_barcode_check_kernel<<<igrid(ctx, nw), 256, 0, st>>>(nw, base, d_text, slot_of, fidx.u32(), fp.bo, fp.bl, hlen.u32(),
-                                                                (const char*)arena.ptr, (const unsigned long long*)soff.ptr, fp.flags + 1);
+    ingest_key_claim_kernel<<<igrid(ctx, nw), 256, 0, st>>>(nw, base, d_text, slot_of, id.u32(), pl.bo, pl.bl, wpos, used,
+                                                            (char*)arena.ptr, (unsigned long long*)soff.ptr, byte0,
+                                                            (unsigned long long*)first_byte.ptr);
+    ingest_key_check_kernel<<<igrid(ctx, nw), 256, 0, st>>>(nw, base, d_text, slot_of, id.u32(), pl.bo, pl.bl, klen.u32(),
+                                                            (const char*)arena.ptr, (const unsigned long long*)soff.ptr, pl.flags + 1);
     ctx->launches += 2;
     uint32_t collision = 0;
-    GT_CUDA(cudaMemcpyAsync(&collision, fp.flags + 1, 4, cudaMemcpyDeviceToHost, st));
+    GT_CUDA(cudaMemcpyAsync(&collision, pl.flags + 1, 4, cudaMemcpyDeviceToHost, st));
     GT_CUDA(cudaStreamSynchronize(st));  // the window's text may be overwritten after this
-    if (collision) return fail(GTGPU_ERR_UNSUPPORTED, who + ": two barcodes share a 64-bit hash; use " + array_entry);
+    if (collision) return fail(GTGPU_ERR_UNSUPPORTED, who + ": two " + keys + " share a 64-bit hash; use " + array_entry);
     used += bytes;
     distinct += tail[2];
     n += nw;
     return GTGPU_OK;
 }
 
-int32_t FragBarcodeTable::finish(gtgpu_ctx* ctx, uint32_t* n_kept, BufPtr* out_names, BufPtr* out_name_offsets, BufPtr* out_spans) {
+int32_t KeyTable::finish(gtgpu_ctx* ctx, uint32_t* n_kept, BufPtr* out_names, BufPtr* out_name_offsets, BufPtr* out_spans) {
     cudaStream_t st = ctx->stream;
-    uint64_t kept = 0, blob_bytes = 0;
+    uint32_t kept = 0;
+    uint64_t blob_bytes = 0;
     char* d_blob = nullptr;
     unsigned long long* d_noff = nullptr;
     uint32_t* d_spans = nullptr;
     if (n) {
-        uint32_t *d_keep, *d_rank;
-        unsigned long long *d_alen, *d_klen, *d_aoff, *d_boff;
+        // the kept keys' first appearances, sorted: key i of that order gets id i
+        uint32_t *k_a, *v_a, *k_b, *v_b, *d_cnt;
         void* d_tmp;
-        GT_TRY(ctx->scratch_get(SC_ING_0, n * 4, (void**)&d_keep));
-        GT_TRY(ctx->scratch_get(SC_ING_1, n * 4, (void**)&d_rank));
-        GT_TRY(ctx->scratch_get(SC_ING_2, n * 8, (void**)&d_alen));
-        GT_TRY(ctx->scratch_get(SC_ING_5, n * 8, (void**)&d_klen));
-        GT_TRY(ctx->scratch_get(SC_ING_3, n * 8, (void**)&d_aoff));
-        GT_TRY(ctx->scratch_get(SC_ING_4, n * 8, (void**)&d_boff));
-        GT_TRY(ctx->scratch_get(SC_IN3_START, exclusive_scan_temp_bytes(n, 8), &d_tmp));
-        GT_TRY(bc.reserve(n * 4, 0, st));
-        ingest_barcode_keep_kernel<<<igrid(ctx, n), 256, 0, st>>>(n, keep_all, fidx.u32(), known.u32(), hlen.u32(), d_keep, d_alen,
-                                                                  d_klen);
+        GT_TRY(ctx->scratch_get(SC_ING_0, distinct * 4, (void**)&k_a));
+        GT_TRY(ctx->scratch_get(SC_ING_1, distinct * 4, (void**)&v_a));
+        GT_TRY(ctx->scratch_get(SC_ING_2, distinct * 4, (void**)&k_b));
+        GT_TRY(ctx->scratch_get(SC_ING_3, distinct * 4, (void**)&v_b));
+        GT_TRY(ctx->scratch_get(SC_MISC, 64, (void**)&d_cnt));
+        GT_CUDA(cudaMemsetAsync(d_cnt, 0, 4, st));
+        ingest_key_kept_kernel<<<igrid(ctx, cap), 256, 0, st>>>(cap, (const unsigned long long*)hash.ptr, first.u32(), known.u32(), k_a,
+                                                                v_a, d_cnt);
         ctx->launches++;
-        GT_TRY(exclusive_scan<uint32_t>(ctx, d_keep, d_rank, n, d_tmp));
-        GT_TRY(exclusive_scan<unsigned long long>(ctx, d_alen, d_aoff, n, d_tmp));
-        GT_TRY(exclusive_scan<unsigned long long>(ctx, d_klen, d_boff, n, d_tmp));
-        uint32_t t32[2];
-        unsigned long long t64[2];
-        GT_CUDA(cudaMemcpyAsync(&t32[0], d_rank + n - 1, 4, cudaMemcpyDeviceToHost, st));
-        GT_CUDA(cudaMemcpyAsync(&t32[1], d_keep + n - 1, 4, cudaMemcpyDeviceToHost, st));
-        GT_CUDA(cudaMemcpyAsync(&t64[0], d_boff + n - 1, 8, cudaMemcpyDeviceToHost, st));
-        GT_CUDA(cudaMemcpyAsync(&t64[1], d_klen + n - 1, 8, cudaMemcpyDeviceToHost, st));
+        GT_CUDA(cudaMemcpyAsync(&kept, d_cnt, 4, cudaMemcpyDeviceToHost, st));
         GT_CUDA(cudaStreamSynchronize(st));
-        kept = (uint64_t)t32[0] + t32[1];
-        blob_bytes = t64[0] + t64[1];
-        if (out_spans) {
-            GT_TRY(ctx->scratch_get(SC_FILE_OFFS, kept * 8 + 8, (void**)&d_spans));
-        } else {
-            GT_TRY(ctx->scratch_get(SC_ING_6, blob_bytes + 1, (void**)&d_blob));
-            GT_TRY(ctx->scratch_get(SC_ING_7, (kept + 1) * 8, (void**)&d_noff));
+        GT_TRY(ctx->scratch_get(SC_IN3_START, std::max(radix_sort_temp_bytes(kept), exclusive_scan_temp_bytes(kept, 8)), &d_tmp));
+        if (kept) {
+            int bits = 1, in_b = 0;
+            while (bits < 32 && (1ull << bits) < n) ++bits;
+            GT_TRY(radix_sort_pairs(ctx, kept, k_a, v_a, k_b, v_b, bits, d_tmp, &in_b));
+            if (in_b) { std::swap(k_a, k_b); std::swap(v_a, v_b); }
+            unsigned long long* d_len = nullptr;
+            if (out_spans) {
+                GT_TRY(ctx->scratch_get(SC_FILE_OFFS, (uint64_t)kept * 8 + 8, (void**)&d_spans));
+            } else {
+                GT_TRY(ctx->scratch_get(SC_ING_4, (uint64_t)kept * 8, (void**)&d_len));
+                GT_TRY(ctx->scratch_get(SC_ING_7, ((uint64_t)kept + 1) * 8, (void**)&d_noff));
+            }
+            ingest_key_lengths_kernel<<<igrid(ctx, kept), 256, 0, st>>>(kept, v_a, klen.u32(), (const unsigned long long*)first_byte.ptr,
+                                                                        d_len, d_spans);
+            ctx->launches++;
+            if (!out_spans) {
+                GT_TRY(exclusive_scan<unsigned long long>(ctx, d_len, d_noff, kept, d_tmp));
+                unsigned long long t64[2];
+                GT_CUDA(cudaMemcpyAsync(&t64[0], d_noff + kept - 1, 8, cudaMemcpyDeviceToHost, st));
+                GT_CUDA(cudaMemcpyAsync(&t64[1], d_len + kept - 1, 8, cudaMemcpyDeviceToHost, st));
+                GT_CUDA(cudaStreamSynchronize(st));
+                blob_bytes = t64[0] + t64[1];
+                GT_TRY(ctx->scratch_get(SC_ING_6, blob_bytes + 1, (void**)&d_blob));
+                ingest_key_names_kernel<<<igrid(ctx, kept), 256, 0, st>>>(kept, v_a, klen.u32(), (const unsigned long long*)soff.ptr,
+                                                                          (const char*)arena.ptr, d_noff, d_blob);
+                ctx->launches++;
+            }
         }
-        ingest_barcode_final_kernel<<<igrid(ctx, n), 256, 0, st>>>(n, fidx.u32(), d_keep, d_rank, d_aoff, d_boff, hlen.u32(),
-                                                                   (const char*)arena.ptr, d_blob, d_noff,
-                                                                   (const unsigned long long*)first_byte.ptr, d_spans, bc.u32());
+        ingest_key_ids_kernel<<<igrid(ctx, n), 256, 0, st>>>(n, k_a, kept, id.u32());
         ctx->launches++;
         GT_CUDA(cudaGetLastError());
     }
-    *n_kept = (uint32_t)kept;
+    *n_kept = kept;
     if (out_spans) {
         BufPtr spans;
-        int32_t s = buf_from_device(ctx, d_spans, kept * 2, 4, st, &spans);
-        if (s == GTGPU_ERR_CUDA) return fail(s, who + ": D2H of the barcode spans failed");
+        int32_t s = buf_from_device(ctx, d_spans, (uint64_t)kept * 2, 4, st, &spans);
+        if (s == GTGPU_ERR_CUDA) return fail(s, who + ": D2H of the " + key + " spans failed");
         GT_TRY(s);
-        if (cudaStreamSynchronize(st) != cudaSuccess) return fail(GTGPU_ERR_CUDA, who + ": D2H of the barcode spans failed");
+        if (cudaStreamSynchronize(st) != cudaSuccess) return fail(GTGPU_ERR_CUDA, who + ": D2H of the " + key + " spans failed");
         *out_spans = std::move(spans);
         return GTGPU_OK;
     }
     BufPtr names, offsets;
     int32_t s = buf_from_device(ctx, d_blob, blob_bytes, 1, st, &names);
-    if (s == GTGPU_ERR_CUDA) return fail(s, who + ": D2H of the barcode names failed");
+    if (s == GTGPU_ERR_CUDA) return fail(s, who + ": D2H of the " + key + " names failed");
     GT_TRY(s);
-    s = buf_new(ctx, kept + 1, 8, &offsets);  // the last offset is written on the host
-    if (s == GTGPU_OK && kept && cudaMemcpyAsync(offsets->block.ptr, d_noff, kept * 8, cudaMemcpyDeviceToHost, st) != cudaSuccess)
-        s = fail(GTGPU_ERR_CUDA, who + ": D2H of the barcode name offsets failed");
+    s = buf_new(ctx, (uint64_t)kept + 1, 8, &offsets);  // the last offset is written on the host
+    if (s == GTGPU_OK && kept && cudaMemcpyAsync(offsets->block.ptr, d_noff, (uint64_t)kept * 8, cudaMemcpyDeviceToHost, st) != cudaSuccess)
+        s = fail(GTGPU_ERR_CUDA, who + ": D2H of the " + key + " name offsets failed");
     if (s == GTGPU_OK && cudaStreamSynchronize(st) != cudaSuccess) s = fail(GTGPU_ERR_CUDA, who + ": D2H failed");
     if (s != GTGPU_OK) {
         cudaStreamSynchronize(st);  // the names' copy may still run
@@ -1015,7 +970,7 @@ int32_t FragBarcodeTable::finish(gtgpu_ctx* ctx, uint32_t* n_kept, BufPtr* out_n
 }
 
 // tokenize_fragment_file (fragments.rs:61-82) from a fragment file's text of any size: every window is parsed and its barcodes
-// go into one FragBarcodeTable that keeps every barcode; after the last window the fragment tokenizer core runs once over the
+// go into one KeyTable that keeps every barcode; after the last window the fragment tokenizer core runs once over the
 // accumulated fragments and their dense barcode ids.  With out_spans the barcodes come back as u32 (first byte, length) spans
 // into the text, else as names + u64 name offsets.  The caller holds ctx->mu.
 int32_t tokenize_fragments_file_locked(gtgpu_index* ix, const char* host_text, const char* dev_text, uint64_t n_bytes, uint32_t n_names,
@@ -1023,14 +978,14 @@ int32_t tokenize_fragments_file_locked(gtgpu_index* ix, const char* host_text, c
                                        uint32_t* out_n_barcodes, BufPtr* out_names, BufPtr* out_name_offsets, BufPtr* out_spans,
                                        BufPtr* out_barcode_offsets, BufPtr* out_ids) {
     gtgpu_ctx* ctx = ix->ctx;
-    FragBarcodeTable tab(true, out_spans != nullptr, who, "gtgpu_tokenize_fragments");
+    KeyTable tab(true, out_spans != nullptr, ~0ull, who, "gtgpu_tokenize_fragments", "barcode", "barcodes");
     if (n_bytes) {
         NameTable nt;
         GT_TRY(upload_name_table(ctx, n_names, names, name_offsets, &nt));
         GT_TRY(for_each_window(ctx, host_text, dev_text, n_bytes, who,
                                [&](const char* d, uint64_t nb, uint64_t byte0, uint64_t line0, uint32_t* n_lines) -> int32_t {
-            FragParse fp;
-            GT_TRY(parse_fragments_locked(ctx, d, nb, nt, FRAG_TOKENIZE, &fp));
+            ParsedLines fp;
+            GT_TRY(parse_lines_locked(ctx, d, nb, FRAG_TOKENIZE, nt, BedFilesView{}, &fp));
             *n_lines = fp.n_lines;
             if (fp.bad_line != 0xFFFFFFFFu)
                 return fail(GTGPU_ERR_INVALID, who + ": Invalid fragment file detected at line: " + std::to_string(line0 + fp.bad_line));
@@ -1042,7 +997,7 @@ int32_t tokenize_fragments_file_locked(gtgpu_index* ix, const char* host_text, c
     BufPtr offs, ids;
     GT_TRY(tab.finish(ctx, &n_barcodes, out_names, out_name_offsets, out_spans));
     GT_TRY(buf_new(ctx, (uint64_t)n_barcodes + 1, 8, &offs));
-    GT_TRY(tokenize_fragments_core(ix, tab.n, tab.chr.u32(), tab.start.u32(), tab.end.u32(), tab.bc.u32(), n_barcodes, unk_id,
+    GT_TRY(tokenize_fragments_core(ix, tab.n, tab.chr.u32(), tab.start.u32(), tab.end.u32(), tab.id.u32(), n_barcodes, unk_id,
                                    (uint64_t*)offs->block.ptr, &ids));
     *out_n_barcodes = n_barcodes;
     *out_barcode_offsets = std::move(offs);
@@ -1051,81 +1006,8 @@ int32_t tokenize_fragments_file_locked(gtgpu_index* ix, const char* host_text, c
 }
 
 // ---- the BED files of an IGD database: region lines of many files, chromosome names discovered on the device ------------------
-// Name table: open addressing on the 64-bit FNV-1a hash of a chromosome name, NAME_SLOTS slots (an assembly names 25 to ~1e5
-// contigs).  Every record finds or claims its name's slot and lowers the slot's first appearance to its own record index; that
-// head copies the name's bytes to an arena, every later record compares its bytes with them (a 64-bit hash collision would merge
-// two names).  A record's chr column holds its slot until the last window, when the slots are numbered in first-appearance order.
-constexpr uint32_t NAME_SLOTS = 1u << 19, MAX_NAMES = NAME_SLOTS / 2;
-
-__global__ void ingest_name_insert_kernel(uint32_t n, const unsigned long long* __restrict__ h, unsigned long long* keys,
-                                          uint32_t* first, uint32_t* __restrict__ slot_of, uint32_t base, uint32_t* __restrict__ full) {
-    const uint32_t stride = gridDim.x * blockDim.x;
-    for (uint32_t k = blockIdx.x * blockDim.x + threadIdx.x; k < n; k += stride) {
-        const unsigned long long key = h[k];
-        uint32_t slot = (uint32_t)((key * 0x9E3779B97F4A7C15ull) >> 32) & (NAME_SLOTS - 1), probes = 0;
-        for (;;) {
-            unsigned long long prev = keys[slot];  // a set key never changes: only an empty slot needs the CAS
-            if (prev == 0ull) prev = atomicCAS(keys + slot, 0ull, key);
-            if (prev == 0ull || prev == key) break;
-            slot = (slot + 1) & (NAME_SLOTS - 1);
-            if (++probes == NAME_SLOTS) {  // more names than slots: reported, never spun on
-                atomicOr(full, 1u);
-                slot = NAME_SLOTS;
-                break;
-            }
-        }
-        // consecutive records mostly share a chromosome: the first lane of each group of equal slots lowers the first appearance
-        const unsigned same = __match_any_sync(__activemask(), slot);
-        if (slot < NAME_SLOTS && (threadIdx.x & 31) == (unsigned)(__ffs(same) - 1) && first[slot] > base + k) atomicMin(first + slot, base + k);
-        slot_of[k] = slot;
-    }
-}
-
-// counters[0] = arena bytes claimed so far, counters[1] = distinct names
-__global__ void ingest_name_heads_kernel(uint32_t n, uint32_t base, const uint32_t* __restrict__ slot_of, const uint32_t* __restrict__ first,
-                                         const uint32_t* __restrict__ len, uint32_t* __restrict__ nlen, unsigned long long* __restrict__ soff,
-                                         unsigned long long* __restrict__ counters) {
-    const uint32_t stride = gridDim.x * blockDim.x;
-    for (uint32_t k = blockIdx.x * blockDim.x + threadIdx.x; k < n; k += stride) {
-        const uint32_t s = slot_of[k];
-        if (s < NAME_SLOTS && first[s] == base + k) {
-            nlen[s] = len[k];
-            soff[s] = atomicAdd(counters, (unsigned long long)len[k]);
-            atomicAdd(counters + 1, 1ull);
-        }
-    }
-}
-
-__global__ void ingest_name_claim_kernel(uint32_t n, uint32_t base, const char* __restrict__ text, const uint32_t* __restrict__ slot_of,
-                                         const uint32_t* __restrict__ first, const uint32_t* __restrict__ off, const uint32_t* __restrict__ len,
-                                         const unsigned long long* __restrict__ soff, char* __restrict__ arena) {
-    const uint32_t stride = gridDim.x * blockDim.x;
-    for (uint32_t k = blockIdx.x * blockDim.x + threadIdx.x; k < n; k += stride) {
-        const uint32_t s = slot_of[k];
-        if (first[s] != base + k) continue;
-        for (uint32_t i = 0; i < len[k]; ++i) arena[soff[s] + i] = text[off[k] + i];
-    }
-}
-
-__global__ void ingest_name_check_kernel(uint32_t n, uint32_t base, const char* __restrict__ text, const uint32_t* __restrict__ slot_of,
-                                         const uint32_t* __restrict__ first, const uint32_t* __restrict__ off, const uint32_t* __restrict__ len,
-                                         const uint32_t* __restrict__ nlen, const unsigned long long* __restrict__ soff,
-                                         const char* __restrict__ arena, uint32_t* __restrict__ collision) {
-    const uint32_t stride = gridDim.x * blockDim.x;
-    for (uint32_t k = blockIdx.x * blockDim.x + threadIdx.x; k < n; k += stride) {
-        const uint32_t s = slot_of[k];
-        if (first[s] == base + k) continue;
-        const uint64_t p = soff[s];
-        bool same = nlen[s] == len[k];
-        for (uint32_t i = 0; same && i < len[k]; ++i) same = arena[p + i] == text[off[k] + i];
-        if (!same) *collision = 1;
-    }
-}
-
-__global__ void ingest_name_ids_kernel(uint64_t n, const uint32_t* __restrict__ id_of_slot, uint32_t* __restrict__ chr) {
-    const uint64_t stride = (uint64_t)gridDim.x * blockDim.x;
-    for (uint64_t g = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x; g < n; g += stride) chr[g] = id_of_slot[chr[g]];
-}
+// The names go through a KeyTable that keeps every name (an assembly names 25 to ~1e5 contigs; at most MAX_CHROM_NAMES).
+constexpr uint64_t MAX_CHROM_NAMES = 1u << 18;
 
 // records are in file order: file f's records start at the first record whose file is >= f
 __global__ void ingest_file_record_offsets_kernel(uint64_t n_files, const uint32_t* __restrict__ file, uint64_t n,
@@ -1146,27 +1028,15 @@ int32_t parse_bed_files_locked(gtgpu_ctx* ctx, const char* host_text, const char
                                const std::string& who, BedFilesRecords* out) {
     cudaStream_t st = ctx->stream;
     const uint64_t n_bytes = file_offsets[n_files];
-    DevMem d_fo, d_first_line, d_fs, keys, first, soff, nlen, arena, counters;
+    DevMem d_fo, d_first_line, d_fs;
     GT_TRY(d_fo.reserve((n_files + 1) * 8, 0, st));
     GT_TRY(d_first_line.reserve(std::max<uint64_t>(n_files, 1) * 8, 0, st));
-    GT_TRY(keys.reserve((size_t)NAME_SLOTS * 8, 0, st));
-    GT_TRY(first.reserve((size_t)NAME_SLOTS * 4, 0, st));
-    GT_TRY(soff.reserve((size_t)NAME_SLOTS * 8, 0, st));
-    GT_TRY(nlen.reserve((size_t)NAME_SLOTS * 4, 0, st));
-    GT_TRY(counters.reserve(32, 0, st));
     GT_CUDA(cudaMemcpyAsync(d_fo.ptr, file_offsets, (n_files + 1) * 8, cudaMemcpyHostToDevice, st));
-    GT_CUDA(cudaMemsetAsync(keys.ptr, 0, (size_t)NAME_SLOTS * 8, st));
-    GT_CUDA(cudaMemsetAsync(first.ptr, 0xFF, (size_t)NAME_SLOTS * 4, st));
-    GT_CUDA(cudaMemsetAsync(counters.ptr, 0, 32, st));
     GT_CUDA(cudaStreamSynchronize(st));  // file_offsets is the caller's
-    unsigned long long* cnt = (unsigned long long*)counters.ptr;  // [0] arena bytes, [1] names, [2] table full / collision flags
-    uint32_t* d_full = (uint32_t*)(cnt + 2);
-    uint64_t used = 0;
-    BedFilesRecords& r = *out;
-    r.n = 0;
+    KeyTable tab(true, false, MAX_CHROM_NAMES, who, "gtgpu_igd_build", "chromosome", "chromosome names");
     std::vector<uint32_t> fs;  // the window's file starts that are not its first byte (window-relative)
     GT_TRY(for_each_window(ctx, host_text, dev_text, n_bytes, who,
-                           [&](const char* d, uint64_t nb, uint64_t byte0, uint64_t line0, uint32_t* n_lines_out) -> int32_t {
+                           [&](const char* d, uint64_t nb, uint64_t byte0, uint64_t line0, uint32_t* n_lines) -> int32_t {
         fs.clear();
         for (const uint64_t* f = std::upper_bound(file_offsets, file_offsets + n_files + 1, byte0);
              f < file_offsets + n_files + 1 && *f < byte0 + nb; ++f)
@@ -1175,57 +1045,21 @@ int32_t parse_bed_files_locked(gtgpu_ctx* ctx, const char* host_text, const char
             GT_TRY(d_fs.reserve(fs.size() * 4, 0, st));
             GT_CUDA(cudaMemcpyAsync(d_fs.ptr, fs.data(), fs.size() * 4, cudaMemcpyHostToDevice, st));
         }
-        uint32_t *d_nl, n_breaks, n_lines;
-        GT_TRY(line_breaks_locked(ctx, d, nb, d_fs.u32(), (uint32_t)fs.size(), &n_breaks, &n_lines, &d_nl));
-        *n_lines_out = n_lines;
-        // ---- parse + compact (the compaction of the fragment parse carries the same six columns) --------------------------------
-        const size_t lb = (size_t)n_lines * 4 + 8;
-        uint32_t *d_keep, *d_pos, *p_file, *p_start, *p_end, *p_off, *p_len, *o_file, *o_start, *o_end, *o_off, *o_len, *d_flags;
-        unsigned long long *p_h, *o_h;
-        void* d_tmp;
-        GT_TRY(ctx->scratch_get(SC_IN3_START, exclusive_scan_temp_bytes(n_lines, 4), &d_tmp));
-        GT_TRY(ctx->scratch_get(SC_ING_0, lb, (void**)&d_keep));
-        GT_TRY(ctx->scratch_get(SC_ING_1, lb, (void**)&d_pos));
-        GT_TRY(ctx->scratch_get(SC_IN2_CHR, lb, (void**)&p_file));
-        GT_TRY(ctx->scratch_get(SC_IN2_START, lb, (void**)&p_start));
-        GT_TRY(ctx->scratch_get(SC_IN2_END, lb, (void**)&p_end));
-        GT_TRY(ctx->scratch_get(SC_CHR, lb, (void**)&o_file));
-        GT_TRY(ctx->scratch_get(SC_START, lb, (void**)&o_start));
-        GT_TRY(ctx->scratch_get(SC_END, lb, (void**)&o_end));
-        GT_TRY(ctx->scratch_get(SC_ING_2, lb * 2, (void**)&p_h));
-        GT_TRY(ctx->scratch_get(SC_ING_3, lb, (void**)&p_off));
-        GT_TRY(ctx->scratch_get(SC_ING_4, lb, (void**)&p_len));
-        GT_TRY(ctx->scratch_get(SC_ING_5, lb * 2, (void**)&o_h));
-        GT_TRY(ctx->scratch_get(SC_ING_6, lb, (void**)&o_off));
-        GT_TRY(ctx->scratch_get(SC_ING_7, lb, (void**)&o_len));
-        GT_TRY(ctx->scratch_get(SC_MISC, 64, (void**)&d_flags));  // [0] first malformed line, [1] name collision
-        const uint32_t init[2] = {0xFFFFFFFFu, 0u};
-        GT_CUDA(cudaMemcpyAsync(d_flags, init, 8, cudaMemcpyHostToDevice, st));
         BedFilesView fv;
         fv.file_offsets = (const unsigned long long*)d_fo.ptr;
         fv.n_files = n_files;
         fv.byte0 = byte0;
         fv.line0 = line0;
         fv.first_line = (unsigned long long*)d_first_line.ptr;
-        fv.name_hash = p_h;
-        fv.name_off = p_off;
-        fv.name_len = p_len;
-        ingest_parse_lines_kernel<true><<<igrid(ctx, n_lines), 256, 0, st>>>(n_lines, n_breaks, nb, d, d_nl, NameTable{}, d_keep, p_file,
-                                                                             p_start, p_end, d_flags, fv);
-        ctx->launches++;
-        GT_TRY(exclusive_scan<uint32_t>(ctx, d_keep, d_pos, n_lines, d_tmp));
-        ingest_compact_fragments_kernel<<<igrid(ctx, n_lines), 256, 0, st>>>(n_lines, d_keep, d_pos, p_file, p_start, p_end, p_h, p_off,
-                                                                             p_len, o_file, o_start, o_end, o_h, o_off, o_len);
-        ctx->launches++;
-        uint32_t tail[3];
-        GT_CUDA(cudaMemcpyAsync(&tail[0], d_pos + n_lines - 1, 4, cudaMemcpyDeviceToHost, st));
-        GT_CUDA(cudaMemcpyAsync(&tail[1], d_keep + n_lines - 1, 4, cudaMemcpyDeviceToHost, st));
-        GT_CUDA(cudaMemcpyAsync(&tail[2], d_flags, 4, cudaMemcpyDeviceToHost, st));
-        GT_CUDA(cudaStreamSynchronize(st));
-        if (tail[2] != 0xFFFFFFFFu) {  // the file of the first malformed line and the line's number in that file
-            const uint32_t li = tail[2];
+        fv.fstart = d_fs.u32();
+        fv.n_fstart = (uint32_t)fs.size();
+        ParsedLines pl;
+        GT_TRY(parse_lines_locked(ctx, d, nb, BED_FILE_LINES, NameTable{}, fv, &pl));
+        *n_lines = pl.n_lines;
+        if (pl.bad_line != 0xFFFFFFFFu) {  // the file of the first malformed line and the line's number in that file
+            const uint32_t li = pl.bad_line;
             uint32_t a = 0;
-            if (li) GT_CUDA(cudaMemcpy(&a, d_nl + li - 1, 4, cudaMemcpyDeviceToHost));
+            if (li) GT_CUDA(cudaMemcpy(&a, pl.breaks + li - 1, 4, cudaMemcpyDeviceToHost));
             const uint64_t pos = byte0 + (li ? a + 1ull : 0ull);
             const uint64_t f = (uint64_t)(std::upper_bound(file_offsets, file_offsets + n_files, pos) - file_offsets) - 1;
             unsigned long long fl = 0;
@@ -1233,40 +1067,15 @@ int32_t parse_bed_files_locked(gtgpu_ctx* ctx, const char* host_text, const char
             return fail(GTGPU_ERR_INVALID, who + ": file " + std::to_string(f) + ", line " + std::to_string(line0 + li - fl + 1) +
                                                ": cannot parse start / end position (RegionParseError)");
         }
-        const uint32_t nw = tail[0] + tail[1];
-        if (nw == 0) return GTGPU_OK;
-        if (r.n + nw >= 0xFFFFFFFFull) return fail(GTGPU_ERR_UNSUPPORTED, who + ": 2^32 - 1 region lines or more");
-        // ---- append the window's records; their names go through the table -------------------------------------------------
-        const uint32_t base = (uint32_t)r.n;
-        const size_t need = (size_t)(r.n + nw) * 4, have = (size_t)r.n * 4;
-        for (DevMem* m : {&r.chr, &r.start, &r.end, &r.file}) GT_TRY(m->reserve(need, have, st));
-        GT_CUDA(cudaMemcpyAsync(r.start.u32() + base, o_start, (size_t)nw * 4, cudaMemcpyDeviceToDevice, st));
-        GT_CUDA(cudaMemcpyAsync(r.end.u32() + base, o_end, (size_t)nw * 4, cudaMemcpyDeviceToDevice, st));
-        GT_CUDA(cudaMemcpyAsync(r.file.u32() + base, o_file, (size_t)nw * 4, cudaMemcpyDeviceToDevice, st));
-        uint32_t* slot_of = r.chr.u32() + base;
-        ingest_name_insert_kernel<<<igrid(ctx, nw), 256, 0, st>>>(nw, o_h, (unsigned long long*)keys.ptr, first.u32(), slot_of, base, d_full);
-        ingest_name_heads_kernel<<<igrid(ctx, nw), 256, 0, st>>>(nw, base, slot_of, first.u32(), o_len, nlen.u32(),
-                                                                 (unsigned long long*)soff.ptr, cnt);
-        ctx->launches += 2;
-        unsigned long long c[3];
-        GT_CUDA(cudaMemcpyAsync(c, cnt, 24, cudaMemcpyDeviceToHost, st));
-        GT_CUDA(cudaStreamSynchronize(st));
-        if ((uint32_t)c[2] || c[1] > MAX_NAMES)
-            return fail(GTGPU_ERR_UNSUPPORTED, who + ": more than " + std::to_string(MAX_NAMES) + " distinct chromosome names");
-        GT_TRY(arena.reserve(c[0] + 1, used, st));
-        ingest_name_claim_kernel<<<igrid(ctx, nw), 256, 0, st>>>(nw, base, d, slot_of, first.u32(), o_off, o_len,
-                                                                 (const unsigned long long*)soff.ptr, (char*)arena.ptr);
-        ingest_name_check_kernel<<<igrid(ctx, nw), 256, 0, st>>>(nw, base, d, slot_of, first.u32(), o_off, o_len, nlen.u32(),
-                                                                 (const unsigned long long*)soff.ptr, (const char*)arena.ptr, d_flags + 1);
-        ctx->launches += 2;
-        uint32_t collision = 0;
-        GT_CUDA(cudaMemcpyAsync(&collision, d_flags + 1, 4, cudaMemcpyDeviceToHost, st));
-        GT_CUDA(cudaStreamSynchronize(st));  // the window's text may be overwritten after this
-        if (collision) return fail(GTGPU_ERR_UNSUPPORTED, who + ": two chromosome names share a 64-bit hash; use gtgpu_igd_build");
-        used = c[0];
-        r.n += nw;
-        return GTGPU_OK;
+        if (pl.n && tab.n + pl.n >= 0xFFFFFFFFull) return fail(GTGPU_ERR_UNSUPPORTED, who + ": 2^32 - 1 region lines or more");
+        return tab.add_window(ctx, d, byte0, pl, 0);
     }));
+    // the table's chr column holds every record's file
+    BedFilesRecords& r = *out;
+    r.n = tab.n;
+    r.file.swap(tab.chr);
+    r.start.swap(tab.start);
+    r.end.swap(tab.end);
     // ---- every file has a region line; records per file ---------------------------------------------------------------------
     r.file_offsets.assign(n_files + 1, 0);
     if (n_files) {
@@ -1283,35 +1092,9 @@ int32_t parse_bed_files_locked(gtgpu_ctx* ctx, const char* host_text, const char
             if (r.file_offsets[f + 1] == r.file_offsets[f])
                 return fail(GTGPU_ERR_INVALID, who + ": file " + std::to_string(f) + ": Corrupted file. 0 regions found");
     }
-    // ---- chromosome ids in first-appearance order; the records' slots become ids ----------------------------------------------
-    std::vector<unsigned long long> h_keys(NAME_SLOTS), h_soff(NAME_SLOTS);
-    std::vector<uint32_t> h_first(NAME_SLOTS), h_nlen(NAME_SLOTS), id_of_slot(NAME_SLOTS, 0), slots;
-    std::string arena_bytes(used, '\0');
-    GT_CUDA(cudaMemcpyAsync(h_keys.data(), keys.ptr, (size_t)NAME_SLOTS * 8, cudaMemcpyDeviceToHost, st));
-    GT_CUDA(cudaMemcpyAsync(h_soff.data(), soff.ptr, (size_t)NAME_SLOTS * 8, cudaMemcpyDeviceToHost, st));
-    GT_CUDA(cudaMemcpyAsync(h_first.data(), first.ptr, (size_t)NAME_SLOTS * 4, cudaMemcpyDeviceToHost, st));
-    GT_CUDA(cudaMemcpyAsync(h_nlen.data(), nlen.ptr, (size_t)NAME_SLOTS * 4, cudaMemcpyDeviceToHost, st));
-    if (used) GT_CUDA(cudaMemcpyAsync(&arena_bytes[0], arena.ptr, used, cudaMemcpyDeviceToHost, st));
-    GT_CUDA(cudaStreamSynchronize(st));
-    for (uint32_t s = 0; s < NAME_SLOTS; ++s)
-        if (h_keys[s]) slots.push_back(s);
-    std::sort(slots.begin(), slots.end(), [&](uint32_t a, uint32_t b) { return h_first[a] < h_first[b]; });
-    r.names.clear();
-    r.name_offsets.assign(1, 0);
-    for (uint32_t id = 0; id < slots.size(); ++id) {
-        id_of_slot[slots[id]] = id;
-        r.names.append(arena_bytes, h_soff[slots[id]], h_nlen[slots[id]]);
-        r.name_offsets.push_back(r.names.size());
-    }
-    if (r.n) {
-        DevMem d_ids;
-        GT_TRY(d_ids.reserve((size_t)NAME_SLOTS * 4, 0, st));
-        GT_CUDA(cudaMemcpyAsync(d_ids.ptr, id_of_slot.data(), (size_t)NAME_SLOTS * 4, cudaMemcpyHostToDevice, st));
-        ingest_name_ids_kernel<<<igrid(ctx, r.n), 256, 0, st>>>(r.n, d_ids.u32(), r.chr.u32());
-        ctx->launches++;
-        GT_CUDA(cudaGetLastError());
-        GT_CUDA(cudaStreamSynchronize(st));  // id_of_slot is pageable
-    }
+    // ---- chromosome ids in first-appearance order ----------------------------------------------------------------------------
+    GT_TRY(tab.finish(ctx, &r.n_names, &r.names, &r.name_offsets));
+    r.chr.swap(tab.id);
     return GTGPU_OK;
 }
 

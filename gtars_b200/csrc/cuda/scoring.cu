@@ -390,8 +390,8 @@ static int32_t score_matrix_text_locked(gtgpu_index* ix, const char* host_text, 
         GT_TRY(ctx->scratch_get(SC_FILE_OFFS, 16, (void**)&d_fo));
         GT_TRY(for_each_window(ctx, host_text, dev_text, n_bytes, who,
                                [&](const char* d, uint64_t nb, uint64_t, uint64_t line0, uint32_t* n_lines) -> int32_t {
-            FragParse fp;
-            GT_TRY(parse_fragments_locked(ctx, d, nb, nt, FRAG_SCORE_MATRIX, &fp));
+            ParsedLines fp;
+            GT_TRY(parse_lines_locked(ctx, d, nb, FRAG_SCORE_MATRIX, nt, BedFilesView{}, &fp));
             *n_lines = fp.n_lines;
             if (fp.bad_line != 0xFFFFFFFFu) return parse_error(who, line0 + fp.bad_line);
             total += fp.n;
@@ -414,14 +414,14 @@ static int32_t score_barcodes_text_locked(gtgpu_index* ix, const char* host_text
                                           gtgpu_buf** out_names, gtgpu_buf** out_name_offsets, gtgpu_buf** out_barcode_offsets,
                                           gtgpu_buf** out_peaks, gtgpu_buf** out_counts, const std::string& who) {
     gtgpu_ctx* ctx = ix->ctx;
-    FragBarcodeTable tab(false, false, who, "gtgpu_score_barcodes");
+    KeyTable tab(false, false, ~0ull, who, "gtgpu_score_barcodes", "barcode", "barcodes");
     if (n_bytes) {
         NameTable nt;
         GT_TRY(upload_name_table(ctx, n_names, names, name_offsets, &nt));
         GT_TRY(for_each_window(ctx, host_text, dev_text, n_bytes, who,
                                [&](const char* d, uint64_t nb, uint64_t byte0, uint64_t line0, uint32_t* n_lines) -> int32_t {
-            FragParse fp;
-            GT_TRY(parse_fragments_locked(ctx, d, nb, nt, FRAG_SCORE_BARCODES, &fp));
+            ParsedLines fp;
+            GT_TRY(parse_lines_locked(ctx, d, nb, FRAG_SCORE_BARCODES, nt, BedFilesView{}, &fp));
             *n_lines = fp.n_lines;
             if (fp.bad_line != 0xFFFFFFFFu) return parse_error(who, line0 + fp.bad_line);
             if (tab.n + fp.n > 0xFFFFFFFFull) return too_many(who);
@@ -432,7 +432,7 @@ static int32_t score_barcodes_text_locked(gtgpu_index* ix, const char* host_text
     BufPtr nm, no, offs;
     GT_TRY(tab.finish(ctx, &n_kept, &nm, &no));
     GT_TRY(buf_new(ctx, (uint64_t)n_kept + 1, 8, &offs));
-    GT_TRY(score_barcodes_dev_locked(ix, tab.n, tab.chr.u32(), tab.start.u32(), tab.end.u32(), tab.bc.u32(), n_kept,
+    GT_TRY(score_barcodes_dev_locked(ix, tab.n, tab.chr.u32(), tab.start.u32(), tab.end.u32(), tab.id.u32(), n_kept,
                                      (uint64_t*)offs->block.ptr, out_peaks, out_counts));
     *out_n_barcodes = n_kept;
     *out_names = nm.release();

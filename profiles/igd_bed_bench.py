@@ -1,13 +1,14 @@
 """Wall time of loading an IGD database from its BED files: api.Igd.from_bed_files(paths) (text parsed on the device) against
-api.Igd([RegionSet(p) for p in paths]) (host parser), files already in the page cache; plus gtgpu_igd_build on C4-shaped arrays
-for two builds of the library timed alternately.
+api.Igd([RegionSet(p) for p in paths]) (host parser), files already in the page cache; plus gtgpu_igd_build_bed / _gz on the
+same files and gtgpu_igd_build on C4-shaped arrays for two builds of the library timed alternately.
 
     python profiles/igd_bed_bench.py [--sets 10000] [--per-set 20000] [--out profiles/igd_bed_bench.jsonl] [--lib PATH ...]
 
 Workloads: a seeded database of --sets BED files of --per-set regions each (C4's shape at the defaults: 1e4 x 2e4), written
 as plain .bed and as one-member .bed.gz files; both loaders on both forms, with the count matrices of one query batch (64
-sets x 2 000 regions) compared between them.  Then gtgpu_igd_build (ffi.Igd) on 1e4 x 2e4 records through each library given
-with --lib (default: the in-tree one), in alternating child processes.  One JSON line per measurement, each with the card's
+sets x 2 000 regions) compared between them.  Then, through each library given with --lib (default: the in-tree one), in
+alternating child processes: gtgpu_igd_build_bed and _gz (ffi.Igd.from_bed_text / from_bed_gz) on the same files, and
+gtgpu_igd_build (ffi.Igd) on 1e4 x 2e4 records.  One JSON line per measurement, each with the card's
 name and power limit read in the same run.  Files go to a temporary directory that is removed at the end.
 """
 from __future__ import annotations
@@ -55,13 +56,54 @@ def write_set(args):
         f.write(gzip.compress(text, compresslevel=6, mtime=0))
 
 
-def build_child(n_sets, per, reps):
-    """Child process: GTGPU_LIB is set by the parent; best wall time of gtgpu_igd_build over C4-shaped arrays."""
+def child_ffi():
+    """the ffi of the library named by GTGPU_LIB (set by the parent)"""
     import ctypes
     from gtars_b200 import ffi
     exported = ctypes.CDLL(ffi.LIB_PATH)
     for name in [n for n in ffi.SIGNATURES if not hasattr(exported, n)]:  # an older build lacks entry points added since
         del ffi.SIGNATURES[name]
+    return ffi
+
+
+def load_child(tmp, n_sets, reps):
+    """Child process: best wall time of gtgpu_igd_build_bed (the plain files back to back) and gtgpu_igd_build_bed_gz (one
+    member per file) over the files in tmp, with a checksum of one query batch's counts."""
+    from gtars_b200 import synth
+    ffi = child_ffi()
+    paths = [os.path.join(tmp, f"set{i:05d}.bed") for i in range(n_sets)]
+    texts = [open(p, "rb").read() for p in paths]
+    gzs = [open(p + ".gz", "rb").read() for p in paths]
+    text, gz = np.frombuffer(b"".join(texts), dtype=np.uint8), np.frombuffer(b"".join(gzs), dtype=np.uint8)
+    fo = np.cumsum([0] + [len(t) for t in texts]).astype(np.uint64)
+    mo = np.cumsum([0] + [len(g) for g in gzs]).astype(np.uint64)
+    qc, qs, qe = records(64 * 2000, 7)
+    so = np.arange(0, 64 * 2000 + 1, 2000, dtype=np.uint64)
+    ctx = ffi.Context(0)
+    res = {}
+    for fmt, call in (("plain", lambda: ffi.Igd.from_bed_text(ctx, text, fo)),
+                      ("gzip", lambda: ffi.Igd.from_bed_gz(ctx, gz, np.arange(n_sets + 1, dtype=np.uint64), mo))):
+        call()[0].close()                                                # warm-up: modules, allocator
+        best = None
+        for _ in range(reps):
+            t = time.perf_counter()
+            g, names = call()
+            dt = time.perf_counter() - t
+            best = dt if best is None else min(best, dt)
+            if _ < reps - 1:
+                g.close()
+        idx = {n: i for i, n in enumerate(names)}
+        remap = np.array([idx.get(n, 0xFFFFFFFF) for n in synth.CHROM_NAMES[:N_CHROMS]], dtype=np.uint32)
+        cnt = g.count_set_overlaps(so, remap[qc], qs, qe)
+        res[fmt] = dict(wall_s=best, n_records=g.info()["n_records"], names=len(names), counts_sum=int(cnt.sum()))
+        g.close()
+    ctx.close()
+    print(json.dumps(res))
+
+
+def build_child(n_sets, per, reps):
+    """Child process: best wall time of gtgpu_igd_build over C4-shaped arrays."""
+    ffi = child_ffi()
     c, s, e = records(n_sets * per, 1)
     fo = np.arange(n_sets + 1, dtype=np.uint64) * np.uint64(per)
     c = c.astype(np.uint32)
@@ -84,9 +126,13 @@ def main():
     ap.add_argument("--rounds", type=int, default=3, help="alternating rounds of the build comparison")
     ap.add_argument("--only-build", action="store_true", help="run the build comparison only")
     ap.add_argument("--build-child", action="store_true", help=argparse.SUPPRESS)
+    ap.add_argument("--load-child", help=argparse.SUPPRESS)
     args = ap.parse_args()
     if args.build_child:
         build_child(10_000, 20_000, 3)
+        return
+    if args.load_child:
+        load_child(args.load_child, args.sets, 3)
         return
     gpu, power = subprocess.run(["nvidia-smi", "--query-gpu=name,power.limit", "--format=csv,noheader"], capture_output=True,
                                 text=True, check=True).stdout.splitlines()[0].split(", ")
@@ -124,6 +170,14 @@ def main():
                      wall_s=th, equal=bool(np.array_equal(host._count(queries, 1, False), want)))
                 del host
         libs = args.lib or [os.path.join(ROOT, "gtars_b200", "libgtars_gpu.so")]
+        if not args.only_build:
+            for r in range(args.rounds):
+                for lib in libs:
+                    env = dict(os.environ, GTGPU_LIB=os.path.abspath(lib))
+                    res = subprocess.run([sys.executable, os.path.abspath(__file__), "--load-child", tmp, "--sets", str(args.sets)],
+                                         env=env, capture_output=True, text=True, check=True)
+                    for fmt, kv in json.loads(res.stdout.strip().splitlines()[-1]).items():
+                        emit(workload="gtgpu_igd_build_bed", sets=args.sets, per_set=args.per_set, format=fmt, lib=lib, round=r, **kv)
         for r in range(args.rounds):
             for lib in libs:
                 env = dict(os.environ, GTGPU_LIB=os.path.abspath(lib))

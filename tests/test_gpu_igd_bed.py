@@ -394,3 +394,65 @@ def test_multi_device_context_equals_single(ctx):
     two.close()
     one.close()
     multi.close()
+
+
+def gz_members(texts):
+    """one gzip member per text: (bytes, file_members, member_offsets) for ffi.Igd.from_bed_gz"""
+    members = [gzip.compress(t, mtime=0) for t in texts]
+    return b"".join(members), np.arange(len(texts) + 1), np.cumsum([0] + [len(m) for m in members]).astype(np.uint64)
+
+
+def test_names_first_seen_over_many_windows(ctx, monkeypatch):
+    """1e5 distinct chromosome names, first seen all along the text, in windows of 64 KiB (about 100 windows): the name table
+    grows during the call.  Names and counts equal gtgpu_igd_build on the same records with first-appearance ids."""
+    from gtars_b200 import ffi
+    n_names, n_files, per = 100_000, 30, 10_000
+    n = n_files * per
+    rng = np.random.default_rng(21)
+    c = np.arange(n) * n_names // n                                     # every name, first seen in order along the text
+    c[1::3] = (c[1::3] + rng.integers(0, 4, len(c[1::3]))) % n_names  # and some lines a few names ahead
+    s = rng.integers(0, 100_000, n).astype(np.uint32)
+    e = (s + rng.integers(1, 5000, n)).astype(np.uint32)
+    lines = [f"c{a}\t{b}\t{d}\n" for a, b, d in zip(c.tolist(), s.tolist(), e.tolist())]
+    texts = ["".join(lines[f * per:(f + 1) * per]).encode() for f in range(n_files)]
+    u, first = np.unique(c, return_index=True)
+    assert len(u) == n_names
+    order = u[np.argsort(first)]                                        # name of id i, in first-appearance order
+    id_of = np.empty(n_names, dtype=np.uint32)
+    id_of[order] = np.arange(n_names, dtype=np.uint32)
+    ref = ffi.Igd(ctx, np.arange(0, n + 1, per, dtype=np.uint64), n_names, id_of[c], s, e)
+    so = np.arange(0, 64 * 500 + 1, 500, dtype=np.uint64)
+    qc = rng.integers(0, n_names, 64 * 500).astype(np.uint32)
+    qs = rng.integers(0, 100_000, 64 * 500).astype(np.uint32)
+    qe = (qs + rng.integers(1, 20_000, 64 * 500)).astype(np.uint32)
+    fo = np.cumsum([0] + [len(t) for t in texts]).astype(np.uint64)
+    monkeypatch.setenv("GTGPU_INGEST_WINDOW", "65536")
+    for g, names in (ffi.Igd.from_bed_text(ctx, b"".join(texts), fo), ffi.Igd.from_bed_gz(ctx, *gz_members(texts))):
+        assert names == [f"c{v}" for v in order]
+        assert g.info()["n_records"] == ref.info()["n_records"]
+        for fn in ("count_set_overlaps", "count_region_hits"):
+            assert np.array_equal(getattr(g, fn)(so, qc, qs, qe), getattr(ref, fn)(so, qc, qs, qe)), fn
+        g.close()
+    ref.close()
+
+
+def test_name_limit(ctx):
+    """262 144 distinct chromosome names load; one more is GTGPU_ERR_UNSUPPORTED with its message, and the ctx stays usable."""
+    from gtars_b200 import ffi
+    limit = 262_144
+    for n_names in (limit, limit + 1):
+        lines = [f"n{i}\t{i % 1000}\t{i % 1000 + 10}\n" for i in range(n_names)]
+        texts = ["".join(lines[f::4]).encode() for f in range(4)]
+        fo = np.cumsum([0] + [len(t) for t in texts]).astype(np.uint64)
+        for call in (lambda: ffi.Igd.from_bed_text(ctx, b"".join(texts), fo), lambda: ffi.Igd.from_bed_gz(ctx, *gz_members(texts))):
+            if n_names == limit:
+                g, names = call()
+                assert len(names) == limit and names[:3] == ["n0", "n4", "n8"] and g.info()["n_records"] == limit
+                g.close()
+            else:
+                with pytest.raises(ffi.GtarsGpuError) as err:
+                    call()
+                assert err.value.code == 6 and "more than 262144 distinct chromosome names" in str(err.value), str(err.value)
+    g, names = ffi.Igd.from_bed_text(ctx, b"chr1\t1\t5\n", np.array([0, 9], dtype=np.uint64))
+    assert names == ["chr1"]
+    g.close()
