@@ -141,6 +141,16 @@ extern "C" {
                                        start: *const u32, end: *const u32, min_overlap: i32, out: *mut u64) -> i32;
     pub fn gtgpu_igd_count_dev(igd: *mut gtgpu_igd, binary: i32, n: u64, d_set_of: *const u32, d_chr: *const u32,
                                d_start: *const u32, d_end: *const u32, min_overlap: i32, d_out: *mut u64) -> i32;
+    /// count_region_hits (binary = 1) / count_set_overlaps (binary = 0) of query sets given as BED files (set s = text[file_offsets[s],
+    /// file_offsets[s + 1])), parsed on the device; names map through the caller's table.  out: [n_sets x n_files];
+    /// out_set_regions: every set's region lines.
+    pub fn gtgpu_igd_count_bed(igd: *mut gtgpu_igd, binary: i32, n_sets: u64, text: *const c_char, file_offsets: *const u64, n_names: u32,
+                               names: *const u8, name_offsets: *const u32, min_overlap: i32, out: *mut u64,
+                               out_set_regions: *mut u64) -> i32;
+    /// The same from gzip members: set s = members [file_members[s], file_members[s + 1]) of gz / member_offsets.
+    pub fn gtgpu_igd_count_bed_gz(igd: *mut gtgpu_igd, binary: i32, n_sets: u64, file_members: *const u64, n_members: u64, gz: *const u8,
+                                  member_offsets: *const u64, n_names: u32, names: *const u8, name_offsets: *const u32,
+                                  min_overlap: i32, out: *mut u64, out_set_regions: *mut u64) -> i32;
     pub fn gtgpu_comm_unique_id(out_id: *mut u8) -> i32;
     pub fn gtgpu_comm_init(ctx: *mut gtgpu_ctx, world: i32, rank: i32, id: *const u8) -> i32;
     pub fn gtgpu_comm_free(ctx: *mut gtgpu_ctx) -> i32;

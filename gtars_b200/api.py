@@ -4,7 +4,7 @@
     gtars.models.Region / RegionSet     -> Region, RegionSet  (gtars-python/src/models/region_set.rs:445-481)
     gtars_overlaprs MultiChromOverlapper / IndexedRegionSet -> MultiChromOverlapper
     gtars.tokenizers.tokenize_fragment_file                 -> tokenize_fragment_file
-    gtars.lola RegionDB / run_lola (contingency counts)     -> Igd, lola_contingency
+    gtars.lola RegionDB / run_lola (contingency counts)     -> Igd, lola_contingency, lola_contingency_from_bed_files
 
 Every batch method is one call into the C++ layer, which marshals to the C ABI of include/gtars_gpu.h; nothing here
 (or below) computes an overlap on the CPU, and construction fails without a CUDA device.
@@ -65,6 +65,8 @@ def lib():
             "gth_igd_new": (vp, [vp, u64, vp]), "gth_igd_free": (None, [vp]), "gth_igd_num_files": (u64, [vp]),
             "gth_igd_count": (C.c_int, [vp, u64, vp, i32, C.c_int, vp]),
             "gth_lola_contingency": (C.c_int, [vp, u64, vp, vp, i32, vp]),
+            "gth_igd_count_bed_files": (C.c_int, [vp, u64, vp, i32, C.c_int, vp, vp]),
+            "gth_lola_contingency_bed_files": (C.c_int, [vp, u64, vp, cp, i32, vp]),
         }
         for name, (res, args) in sig.items():
             fn = getattr(L, name)
@@ -539,6 +541,18 @@ class Igd:
     def count_region_hits(self, regions, min_overlap=1):
         return [int(x) for x in self._count([regions], min_overlap, False)[0]]
 
+    def count_bed_files(self, paths, min_overlap=1, pairwise=False) -> np.ndarray:
+        """count_region_hits (pairwise: count_set_overlaps) of every BED file of `paths` as one query set, the files' text
+        parsed on the device (gtgpu_igd_count_bed; the gzip bytes inflated there when every path ends in .gz): uint64
+        [len(paths), num_files()], row i == count_region_hits(RegionSet(paths[i]))."""
+        paths = [os.fsencode(p) for p in paths]
+        out = np.zeros((len(paths), self.num_files()), dtype=np.uint64)
+        regions = np.zeros(len(paths), dtype=np.uint64)
+        if lib().gth_igd_count_bed_files(self._h, len(paths), (C.c_char_p * max(len(paths), 1))(*paths), min_overlap,
+                                         1 if pairwise else 0, out.ctypes.data, regions.ctypes.data):
+            _fail()
+        return out
+
 
 def write_igd_file(region_sets, names, path):
     """Igd::from_named_region_sets + Igd::save (igd.rs:285-317, 418-486) without building a device index: `path`
@@ -557,5 +571,16 @@ def lola_contingency(igd: Igd, user_sets, universe, min_overlap=1) -> np.ndarray
     arr = (C.c_void_p * max(len(sets), 1))(*[s._h for s in sets])
     out = np.zeros((len(sets), igd.num_files(), 4), dtype=np.int64)
     if lib().gth_lola_contingency(igd._h, len(sets), arr, uni._h, min_overlap, out.ctypes.data):
+        _fail()
+    return out
+
+
+def lola_contingency_from_bed_files(igd: Igd, user_set_paths, universe_path, min_overlap=1) -> np.ndarray:
+    """lola_contingency(igd, [RegionSet(p) for p in user_set_paths], RegionSet(universe_path)) with the user sets and the
+    universe parsed on the device in one pass (gtgpu_igd_count_bed): int64 [n_user, n_db, 4] = a, b, c, d."""
+    paths = [os.fsencode(p) for p in user_set_paths]
+    out = np.zeros((len(paths), igd.num_files(), 4), dtype=np.int64)
+    if lib().gth_lola_contingency_bed_files(igd._h, len(paths), (C.c_char_p * max(len(paths), 1))(*paths),
+                                            os.fsencode(universe_path), min_overlap, out.ctypes.data):
         _fail()
     return out

@@ -147,7 +147,8 @@ int32_t gtgpu::group_comm_ensure(gtgpu_ctx* g) {
 }
 
 // Database sharded by region set: rank r owns global files [r * cols, min((r+1) * cols, n_files_global)),
-// cols = ceil(n_files_global / world); `igd` was built over exactly those files (possibly none).  `out` may be null (a
+// cols = ceil(n_files_global / world); `igd` was built over exactly those files (possibly none).  chr / start / end may be
+// host memory or device memory of any device (cudaMemcpyDefault); set_offsets is host memory.  `out` may be null (a
 // peer of an in-process group: only the first device returns the matrix); before_collective, when given, runs right
 // before the all-gather is queued (groups use it as a barrier so that no thread is still allocating device memory while
 // another one's collective kernel already waits for it).
@@ -196,10 +197,10 @@ int32_t gtgpu::igd_count_sharded_impl(gtgpu_ctx* ctx, gtgpu_igd* igd, int32_t bi
         GT_TRY(ctx->scratch_get(SC_IN3_CHR, (uint64_t)world * n_sets * cols * 8 + 8, (void**)&d_gather));
         GT_TRY(ctx->scratch_get(SC_IN3_START, n_sets * n_files_global * 8 + 8, (void**)&d_full));
         if (local != cols) GT_TRY(ctx->scratch_get(SC_IN3_END, n_sets * local * 8 + 8, (void**)&d_tmp));
-        if (n) {
-            GT_CUDA(cudaMemcpyAsync(d_chr, chr, n * 4, cudaMemcpyHostToDevice, st));
-            GT_CUDA(cudaMemcpyAsync(d_start, start, n * 4, cudaMemcpyHostToDevice, st));
-            GT_CUDA(cudaMemcpyAsync(d_end, end, n * 4, cudaMemcpyHostToDevice, st));
+        if (n) {  // host arrays, or (a group counting parsed BED files) the first device's columns
+            GT_CUDA(cudaMemcpyAsync(d_chr, chr, n * 4, cudaMemcpyDefault, st));
+            GT_CUDA(cudaMemcpyAsync(d_start, start, n * 4, cudaMemcpyDefault, st));
+            GT_CUDA(cudaMemcpyAsync(d_end, end, n * 4, cudaMemcpyDefault, st));
         }
         GT_CUDA(cudaMemcpyAsync(d_so, set_offsets, (n_sets + 1) * 8, cudaMemcpyHostToDevice, st));
         GT_CUDA(cudaMemsetAsync(d_local, 0, n_sets * cols * 8 + 8, st));

@@ -669,6 +669,22 @@ int32_t igd_count_group(gtgpu_igd* g, bool binary, uint64_t n_sets, const uint64
     });
 }
 
+// The count half of every single-device count: n device-resident queries of g's device (query i in set d_set_of[i]) into a
+// zeroed [n_sets x n_files] matrix (scratch SC_MATRIX), copied to the host's out.  The caller holds ctx->mu.
+static int32_t igd_count_to_host_locked(gtgpu_igd* g, bool binary, uint64_t n_sets, uint64_t n, const uint32_t* d_set,
+                                        const uint32_t* d_chr, const uint32_t* d_start, const uint32_t* d_end, int32_t m, uint64_t* out) {
+    gtgpu_ctx* ctx = g->ctx;
+    cudaStream_t st = ctx->stream;
+    uint64_t* d_out;
+    const uint64_t cells = n_sets * g->n_files;
+    GT_TRY(ctx->scratch_get(SC_MATRIX, cells * 8, (void**)&d_out));
+    GT_CUDA(cudaMemsetAsync(d_out, 0, std::max<uint64_t>(cells * 8, 8), st));
+    GT_TRY(igd_count_dev_locked(g, binary, n, d_set, d_chr, d_start, d_end, m, d_out));
+    if (cells) GT_CUDA(cudaMemcpyAsync(out, d_out, cells * 8, cudaMemcpyDeviceToHost, st));
+    GT_CUDA(cudaStreamSynchronize(st));
+    return GTGPU_OK;
+}
+
 int32_t igd_count_host(gtgpu_igd* g, bool binary, uint64_t n_sets, const uint64_t* set_offsets, const uint32_t* chr,
                        const uint32_t* start, const uint32_t* end, int32_t m, uint64_t* out) {
     if (!g || !set_offsets || !out) return fail(GTGPU_ERR_INVALID, "igd count: null argument");
@@ -681,27 +697,22 @@ int32_t igd_count_host(gtgpu_igd* g, bool binary, uint64_t n_sets, const uint64_
     std::lock_guard<std::mutex> lk(ctx->mu);
     GT_CUDA(cudaSetDevice(ctx->device));
     cudaStream_t st = ctx->stream;
+    // the queries to the device
     uint32_t *d_chr, *d_start, *d_end, *d_set;
-    uint64_t *d_so, *d_out;
+    uint64_t* d_so;
     GT_TRY(ctx->scratch_get(SC_CHR, n * 4, (void**)&d_chr));
     GT_TRY(ctx->scratch_get(SC_START, n * 4, (void**)&d_start));
     GT_TRY(ctx->scratch_get(SC_END, n * 4, (void**)&d_end));
     GT_TRY(ctx->scratch_get(SC_SET_ID, n * 4, (void**)&d_set));
     GT_TRY(ctx->scratch_get(SC_FILE_OFFS, (n_sets + 1) * 8, (void**)&d_so));
-    const uint64_t cells = n_sets * g->n_files;
-    GT_TRY(ctx->scratch_get(SC_MATRIX, cells * 8, (void**)&d_out));
     if (n) {
         GT_CUDA(cudaMemcpyAsync(d_chr, chr, n * 4, cudaMemcpyHostToDevice, st));
         GT_CUDA(cudaMemcpyAsync(d_start, start, n * 4, cudaMemcpyHostToDevice, st));
         GT_CUDA(cudaMemcpyAsync(d_end, end, n * 4, cudaMemcpyHostToDevice, st));
     }
     GT_CUDA(cudaMemcpyAsync(d_so, set_offsets, (n_sets + 1) * 8, cudaMemcpyHostToDevice, st));
-    GT_CUDA(cudaMemsetAsync(d_out, 0, std::max<uint64_t>(cells * 8, 8), st));
     if (n_sets && n) GT_TRY(launch_fill_set_ids(ctx, n_sets, d_so, d_set));
-    GT_TRY(igd_count_dev_locked(g, binary, n, d_set, d_chr, d_start, d_end, m, d_out));
-    if (cells) GT_CUDA(cudaMemcpyAsync(out, d_out, cells * 8, cudaMemcpyDeviceToHost, st));
-    GT_CUDA(cudaStreamSynchronize(st));
-    return GTGPU_OK;
+    return igd_count_to_host_locked(g, binary, n_sets, n, d_set, d_chr, d_start, d_end, m, out);
 }
 
 }  // namespace
@@ -728,4 +739,128 @@ extern "C" int32_t gtgpu_igd_count_dev(gtgpu_igd* igd, int32_t binary, uint64_t 
     std::lock_guard<std::mutex> lk(igd->ctx->mu);
     GT_CUDA(cudaSetDevice(igd->ctx->device));
     return igd_count_dev_locked(igd, binary != 0, n, d_set_of, d_chr, d_start, d_end, min_overlap, d_out);
+} GT_CATCH
+
+// ---- query sets from their BED files' text, parsed on the device ------------------------------------------------------------
+// parse_bed_files_locked numbers the query files' chromosome names in their first appearance; one launch maps every such name
+// to the database's id (the caller's name table, looked up as gtgpu_parse_bed does), one more rewrites every record's chr.
+namespace gtgpu {
+
+__global__ void igd_map_names_kernel(uint32_t n_names, const char* __restrict__ blob, const unsigned long long* __restrict__ offs,
+                                     NameTable nt, uint32_t* __restrict__ map) {
+    const uint32_t stride = gridDim.x * blockDim.x;
+    for (uint32_t i = blockIdx.x * blockDim.x + threadIdx.x; i < n_names; i += stride) {
+        const char* s = blob + offs[i];
+        const uint32_t len = (uint32_t)(offs[i + 1] - offs[i]);
+        map[i] = nt.lookup(fnv1a64(s, len), s, len);
+    }
+}
+
+__global__ void igd_remap_chr_kernel(uint64_t n, const uint32_t* __restrict__ map, uint32_t* __restrict__ chr) {
+    const uint64_t stride = (uint64_t)gridDim.x * blockDim.x;
+    for (uint64_t i = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += stride) chr[i] = map[chr[i]];
+}
+
+}  // namespace gtgpu
+
+// The query sets' records (set s = file s of the text, host_text or dev_text, file_offsets in bytes), their chr already in the
+// ids of the caller's names (GTGPU_UNKNOWN_CHROM for a name the database lacks).  The caller holds ctx->mu.
+static int32_t igd_parse_queries_locked(gtgpu_ctx* ctx, const char* host_text, const char* dev_text, uint64_t n_sets,
+                                        const uint64_t* file_offsets, uint32_t n_names, const char* names, const uint32_t* name_offsets,
+                                        const char* who, BedFilesRecords* r) {
+    GT_TRY(parse_bed_files_locked(ctx, host_text, dev_text, n_sets, file_offsets, who, r));
+    if (r->n == 0) return GTGPU_OK;
+    cudaStream_t st = ctx->stream;
+    NameTable nt;
+    GT_TRY(upload_name_table(ctx, n_names, names, name_offsets, &nt));  // scratch SC_SET_ID
+    const uint64_t blob_bytes = r->names->len;
+    DevMem d_blob, d_offs, d_map;
+    GT_TRY(d_blob.reserve(std::max<uint64_t>(blob_bytes, 1), 0, st));
+    GT_TRY(d_offs.reserve(((uint64_t)r->n_names + 1) * 8, 0, st));
+    GT_TRY(d_map.reserve((uint64_t)r->n_names * 4, 0, st));
+    if (blob_bytes) GT_CUDA(cudaMemcpyAsync(d_blob.ptr, r->names->block.ptr, blob_bytes, cudaMemcpyHostToDevice, st));
+    GT_CUDA(cudaMemcpyAsync(d_offs.ptr, r->name_offsets->block.ptr, ((uint64_t)r->n_names + 1) * 8, cudaMemcpyHostToDevice, st));
+    igd_map_names_kernel<<<grid_for(ctx, r->n_names), 256, 0, st>>>(r->n_names, (const char*)d_blob.ptr,
+                                                                      (const unsigned long long*)d_offs.ptr, nt, d_map.u32());
+    igd_remap_chr_kernel<<<grid_for(ctx, r->n), 256, 0, st>>>(r->n, d_map.u32(), r->chr.u32());
+    ctx->launches += 2;
+    GT_CUDA(cudaGetLastError());
+    GT_CUDA(cudaStreamSynchronize(st));  // the map is freed here, and a count may reuse the name table's scratch
+    return GTGPU_OK;
+}
+
+// The parsed query sets against g.  One device counts the columns where the parse left them; a group runs its sharded count
+// with them as query arrays (each device pulls them from the first one) and gathers the shards' columns.
+static int32_t igd_count_parsed(gtgpu_igd* g, bool binary, uint64_t n_sets, const BedFilesRecords& r, int32_t m, uint64_t* out,
+                                uint64_t* out_set_regions) {
+    gtgpu_ctx* ctx = g->ctx;
+    if (!g->shards.empty()) {
+        const int32_t s = igd_count_group(g, binary, n_sets, r.file_offsets.data(), r.chr.u32(), r.start.u32(), r.end.u32(), m, out);
+        GT_CUDA(cudaSetDevice(ctx->device));  // the parsed records are freed on their device
+        GT_TRY(s);
+    } else {
+        std::lock_guard<std::mutex> lk(ctx->mu);
+        GT_CUDA(cudaSetDevice(ctx->device));
+        GT_TRY(igd_count_to_host_locked(g, binary, n_sets, r.n, r.file.u32(), r.chr.u32(), r.start.u32(), r.end.u32(), m, out));
+    }
+    for (uint64_t s = 0; s < n_sets; ++s) out_set_regions[s] = r.file_offsets[s + 1] - r.file_offsets[s];
+    return GTGPU_OK;
+}
+
+static int32_t igd_count_bed_check(const char* who, gtgpu_igd* igd, uint64_t n_sets, uint32_t n_names, const char* names,
+                                   const uint32_t* name_offsets, int32_t min_overlap, uint64_t* out, uint64_t* out_set_regions) {
+    if (!igd || !out || !out_set_regions || (n_names && (!names || !name_offsets)))
+        return fail(GTGPU_ERR_INVALID, std::string(who) + ": null argument");
+    if (n_sets >= 0xFFFFFFFFull) return fail(GTGPU_ERR_UNSUPPORTED, std::string(who) + ": too many sets");
+    if (min_overlap < 1)
+        return fail(GTGPU_ERR_UNSUPPORTED, std::string(who) + ": min_overlap < 1 depends on the reference's tile layout and is not supported");
+    return GTGPU_OK;
+}
+
+extern "C" int32_t gtgpu_igd_count_bed(gtgpu_igd* igd, int32_t binary, uint64_t n_sets, const char* text, const uint64_t* file_offsets,
+                                       uint32_t n_names, const char* names, const uint32_t* name_offsets, int32_t min_overlap,
+                                       uint64_t* out, uint64_t* out_set_regions) try {
+    GT_TRY(igd_count_bed_check("igd_count_bed", igd, n_sets, n_names, names, name_offsets, min_overlap, out, out_set_regions));
+    if (!file_offsets) return fail(GTGPU_ERR_INVALID, "igd_count_bed: null argument");
+    if (file_offsets[0] != 0) return fail(GTGPU_ERR_INVALID, "igd_count_bed: file_offsets[0] must be 0");
+    for (uint64_t s = 0; s < n_sets; ++s)
+        if (file_offsets[s] > file_offsets[s + 1]) return fail(GTGPU_ERR_INVALID, "igd_count_bed: file_offsets not monotone");
+    if (file_offsets[n_sets] && !text) return fail(GTGPU_ERR_INVALID, "igd_count_bed: null text");
+    if (n_sets == 0) return GTGPU_OK;
+    gtgpu_ctx* ctx = igd->ctx;
+    BedFilesRecords r;
+    {
+        std::lock_guard<std::mutex> lk(ctx->mu);
+        GT_CUDA(cudaSetDevice(ctx->device));
+        GT_TRY(igd_parse_queries_locked(ctx, text, nullptr, n_sets, file_offsets, n_names, names, name_offsets, "igd_count_bed", &r));
+    }
+    return igd_count_parsed(igd, binary != 0, n_sets, r, min_overlap, out, out_set_regions);
+} GT_CATCH
+
+extern "C" int32_t gtgpu_igd_count_bed_gz(gtgpu_igd* igd, int32_t binary, uint64_t n_sets, const uint64_t* file_members,
+                                          uint64_t n_members, const uint8_t* gz, const uint64_t* member_offsets, uint32_t n_names,
+                                          const char* names, const uint32_t* name_offsets, int32_t min_overlap, uint64_t* out,
+                                          uint64_t* out_set_regions) try {
+    GT_TRY(igd_count_bed_check("igd_count_bed_gz", igd, n_sets, n_names, names, name_offsets, min_overlap, out, out_set_regions));
+    if (!file_members) return fail(GTGPU_ERR_INVALID, "igd_count_bed_gz: null argument");
+    GT_TRY(check_members(n_members, gz, member_offsets, "igd_count_bed_gz"));
+    if (file_members[0] != 0 || file_members[n_sets] != n_members)
+        return fail(GTGPU_ERR_INVALID, "igd_count_bed_gz: file_members must run from 0 to n_members");
+    for (uint64_t s = 0; s < n_sets; ++s)
+        if (file_members[s] > file_members[s + 1]) return fail(GTGPU_ERR_INVALID, "igd_count_bed_gz: file_members not monotone");
+    if (n_sets == 0) return GTGPU_OK;
+    gtgpu_ctx* ctx = igd->ctx;
+    BedFilesRecords r;
+    {
+        std::lock_guard<std::mutex> lk(ctx->mu);
+        GT_CUDA(cudaSetDevice(ctx->device));
+        uint8_t* d_text = nullptr;
+        uint64_t n_text = 0;
+        std::vector<uint64_t> text_offsets(n_members + 1), fo(n_sets + 1);
+        GT_TRY(inflate_whole_locked(ctx, n_members, gz, member_offsets, "igd_count_bed_gz", &d_text, &n_text, text_offsets.data()));
+        for (uint64_t s = 0; s <= n_sets; ++s) fo[s] = text_offsets[file_members[s]];
+        GT_TRY(igd_parse_queries_locked(ctx, nullptr, (const char*)d_text, n_sets, fo.data(), n_names, names, name_offsets,
+                                        "igd_count_bed_gz", &r));
+    }
+    return igd_count_parsed(igd, binary != 0, n_sets, r, min_overlap, out, out_set_regions);
 } GT_CATCH

@@ -1146,6 +1146,80 @@ std::unique_ptr<Igd> Igd::from_igd_file(std::shared_ptr<Device> dev, const std::
     return g;
 }
 
+namespace {
+// The bytes of n BED files for one device call.  When every path ends in ".gz" they stay gzip: every file's bytes back to back
+// with their member offsets, for the device inflater.  Otherwise the texts go back to back (".gz" inflated by zlib).
+struct BedFilesBytes {
+    bool gz = false;
+    std::string raw;                                   // gz: the files' gzip bytes
+    std::vector<uint64_t> members{0}, file_members{0};  // gz: member offsets in raw; file f = members [file_members[f], [f + 1])
+    std::unique_ptr<char[]> text;                      // otherwise: the texts, file f = text[file_offsets[f], file_offsets[f + 1])
+    std::vector<uint64_t> file_offsets{0};
+};
+
+BedFilesBytes gather_bed_files(const std::vector<std::string>& paths) {
+    BedFilesBytes b;
+    if (!paths.empty() && std::all_of(paths.begin(), paths.end(), ends_with_gz)) {
+        // one-member .bed.gz files are the common case: every member of every file is inflated on the device in parallel
+        b.gz = true;
+        std::string raw;
+        std::vector<uint64_t> m;
+        for (const auto& p : paths) {
+            read_raw_bytes(p, raw);
+            uint64_t n = 0;
+            gtgpu_gzip_members((const uint8_t*)raw.data(), raw.size(), 0, nullptr, &n);  // count only
+            m.assign(n + 1, 0);
+            check(gtgpu_gzip_members((const uint8_t*)raw.data(), raw.size(), m.size(), m.data(), &n), "gtgpu_gzip_members");
+            for (uint64_t k = 1; k <= n; ++k) b.members.push_back(b.raw.size() + m[k]);
+            b.file_members.push_back(b.members.size() - 1);
+            b.raw += raw;
+        }
+        return b;
+    }
+    // the texts back to back; the library stages them to the device through its own pinned blocks
+    std::vector<std::string> inflated(paths.size());
+    for (size_t f = 0; f < paths.size(); ++f) {
+        uint64_t size = 0;
+        if (ends_with_gz(paths[f])) {
+            inflated[f] = read_file_bytes(paths[f]);
+            size = inflated[f].size();
+        } else {
+            std::ifstream in(paths[f], std::ios::binary | std::ios::ate);
+            if (!in) throw Error("Failed to open file: \"" + paths[f] + "\"");
+            size = (uint64_t)std::max<std::streamsize>(in.tellg(), 0);
+        }
+        b.file_offsets.push_back(b.file_offsets.back() + size);
+    }
+    b.text.reset(new char[std::max<uint64_t>(b.file_offsets.back(), 1)]);
+    for (size_t f = 0; f < paths.size(); ++f) {
+        char* dst = b.text.get() + b.file_offsets[f];
+        const uint64_t size = b.file_offsets[f + 1] - b.file_offsets[f];
+        if (ends_with_gz(paths[f])) {
+            memcpy(dst, inflated[f].data(), size);
+            std::string().swap(inflated[f]);
+        } else if (size) {
+            std::ifstream in(paths[f], std::ios::binary);
+            if (!in || !in.read(dst, (std::streamsize)size)) throw Error("Failed to read file: \"" + paths[f] + "\"");
+        }
+    }
+    return b;
+}
+
+// The library's last error as "fn: message", "file k" in it replaced by the file's path
+[[noreturn]] void throw_naming_path(const char* fn, const std::vector<std::string>& paths) {
+    std::string msg = gtgpu_last_error();
+    const size_t k = msg.find(": file ");
+    size_t b = k == std::string::npos ? k : k + 7;
+    if (b != std::string::npos) {
+        const size_t a = b;
+        while (b < msg.size() && isdigit((unsigned char)msg[b])) ++b;
+        if (b > a && std::stoull(msg.substr(a, b - a)) < paths.size())
+            msg = msg.substr(0, k) + ": \"" + paths[std::stoull(msg.substr(a, b - a))] + "\"" + msg.substr(b);
+    }
+    throw Error(std::string(fn) + ": " + msg);
+}
+}  // namespace
+
 std::unique_ptr<Igd> Igd::from_bed_files(std::shared_ptr<Device> dev, const std::vector<std::string>& paths) {
     std::unique_ptr<Igd> g(new Igd());
     g->dev_ = dev;
@@ -1154,71 +1228,44 @@ std::unique_ptr<Igd> Igd::from_bed_files(std::shared_ptr<Device> dev, const std:
     PinnedResult names, name_offsets;
     int32_t status;
     const char* fn;
-    if (!paths.empty() && std::all_of(paths.begin(), paths.end(), ends_with_gz)) {
-        // one-member .bed.gz files are the common case: every member of every file is inflated on the device in parallel
-        std::string gz, raw;
-        std::vector<uint64_t> members{0}, file_members{0}, m;
-        for (const auto& p : paths) {
-            read_raw_bytes(p, raw);
-            uint64_t n = 0;
-            gtgpu_gzip_members((const uint8_t*)raw.data(), raw.size(), 0, nullptr, &n);  // count only
-            m.assign(n + 1, 0);
-            check(gtgpu_gzip_members((const uint8_t*)raw.data(), raw.size(), m.size(), m.data(), &n), "gtgpu_gzip_members");
-            for (uint64_t k = 1; k <= n; ++k) members.push_back(gz.size() + m[k]);
-            file_members.push_back(members.size() - 1);
-            gz += raw;
-        }
+    const BedFilesBytes b = gather_bed_files(paths);
+    if (b.gz) {
         fn = "gtgpu_igd_build_bed_gz";
-        status = gtgpu_igd_build_bed_gz(dev->ctx(), paths.size(), file_members.data(), members.size() - 1, (const uint8_t*)gz.data(),
-                                        members.data(), &n_chroms, &names.buf, &name_offsets.buf, &g->igd_);
+        status = gtgpu_igd_build_bed_gz(dev->ctx(), paths.size(), b.file_members.data(), b.members.size() - 1, (const uint8_t*)b.raw.data(),
+                                        b.members.data(), &n_chroms, &names.buf, &name_offsets.buf, &g->igd_);
     } else {
-        // the texts back to back; the library stages them to the device through its own pinned blocks
-        std::vector<uint64_t> file_offsets{0};
-        std::vector<std::string> inflated(paths.size());
-        for (size_t f = 0; f < paths.size(); ++f) {
-            uint64_t size = 0;
-            if (ends_with_gz(paths[f])) {
-                inflated[f] = read_file_bytes(paths[f]);
-                size = inflated[f].size();
-            } else {
-                std::ifstream in(paths[f], std::ios::binary | std::ios::ate);
-                if (!in) throw Error("Failed to open file: \"" + paths[f] + "\"");
-                size = (uint64_t)std::max<std::streamsize>(in.tellg(), 0);
-            }
-            file_offsets.push_back(file_offsets.back() + size);
-        }
-        std::unique_ptr<char[]> text(new char[std::max<uint64_t>(file_offsets.back(), 1)]);
-        for (size_t f = 0; f < paths.size(); ++f) {
-            char* dst = text.get() + file_offsets[f];
-            const uint64_t size = file_offsets[f + 1] - file_offsets[f];
-            if (ends_with_gz(paths[f])) {
-                memcpy(dst, inflated[f].data(), size);
-                std::string().swap(inflated[f]);
-            } else if (size) {
-                std::ifstream in(paths[f], std::ios::binary);
-                if (!in || !in.read(dst, (std::streamsize)size)) throw Error("Failed to read file: \"" + paths[f] + "\"");
-            }
-        }
         fn = "gtgpu_igd_build_bed";
-        status = gtgpu_igd_build_bed(dev->ctx(), paths.size(), text.get(), file_offsets.data(), &n_chroms, &names.buf, &name_offsets.buf,
-                                     &g->igd_);
+        status = gtgpu_igd_build_bed(dev->ctx(), paths.size(), b.text.get(), b.file_offsets.data(), &n_chroms, &names.buf,
+                                     &name_offsets.buf, &g->igd_);
     }
-    if (status != GTGPU_OK) {  // "file k" in the library's message becomes the file's path
-        std::string msg = gtgpu_last_error();
-        const size_t k = msg.find(": file ");
-        size_t b = k == std::string::npos ? k : k + 7;
-        if (b != std::string::npos) {
-            const size_t a = b;
-            while (b < msg.size() && isdigit((unsigned char)msg[b])) ++b;
-            if (b > a && std::stoull(msg.substr(a, b - a)) < paths.size())
-                msg = msg.substr(0, k) + ": \"" + paths[std::stoull(msg.substr(a, b - a))] + "\"" + msg.substr(b);
-        }
-        throw Error(std::string(fn) + ": " + msg);
-    }
+    if (status != GTGPU_OK) throw_naming_path(fn, paths);
     const char* blob = (const char*)gtgpu_buf_data(names.buf);
     const uint64_t* noff = (const uint64_t*)gtgpu_buf_data(name_offsets.buf);
     for (uint32_t c = 0; c < n_chroms; ++c) g->cmap_.add(std::string(blob + noff[c], noff[c + 1] - noff[c]));
     return g;
+}
+
+Igd::BedCounts Igd::count_bed_files(const std::vector<std::string>& paths, int32_t min_overlap, bool pairwise) const {
+    if (!igd_) throw Error("count_bed_files needs a database Igd (not from_single_region_set)");
+    BedCounts r;
+    r.matrix.assign(paths.size() * n_files_, 0);
+    r.set_regions.assign(paths.size(), 0);
+    const BedFilesBytes b = gather_bed_files(paths);
+    NameBlob nb(cmap_);
+    int32_t status;
+    const char* fn;
+    if (b.gz) {
+        fn = "gtgpu_igd_count_bed_gz";
+        status = gtgpu_igd_count_bed_gz(igd_, pairwise ? 0 : 1, paths.size(), b.file_members.data(), b.members.size() - 1,
+                                        (const uint8_t*)b.raw.data(), b.members.data(), (uint32_t)cmap_.size(), nb.blob.data(),
+                                        nb.offsets.data(), min_overlap, r.matrix.data(), r.set_regions.data());
+    } else {
+        fn = "gtgpu_igd_count_bed";
+        status = gtgpu_igd_count_bed(igd_, pairwise ? 0 : 1, paths.size(), b.text.get(), b.file_offsets.data(), (uint32_t)cmap_.size(),
+                                     nb.blob.data(), nb.offsets.data(), min_overlap, r.matrix.data(), r.set_regions.data());
+    }
+    if (status != GTGPU_OK) throw_naming_path(fn, paths);
+    return r;
 }
 
 std::array<uint64_t, 4> Igd::info() const {
@@ -1269,25 +1316,45 @@ std::vector<uint64_t> Igd::count_region_hits(const RegionSet& regions, int32_t m
     return count_region_hits_batch({&regions}, min_overlap, false);
 }
 
+namespace {
+// run_lola's tables (enrichment.rs:198-220) from the hit matrix of the user sets with the universe as its last row
+std::vector<std::vector<ContingencyCounts>> contingency_tables(const std::vector<uint64_t>& hits, size_t nf,
+                                                               const std::vector<uint64_t>& user_sizes, uint64_t universe_size) {
+    const uint64_t* universe_hits = hits.data() + user_sizes.size() * nf;
+    std::vector<std::vector<ContingencyCounts>> out(user_sizes.size(), std::vector<ContingencyCounts>(nf));
+    for (size_t u = 0; u < user_sizes.size(); ++u)
+        for (size_t f = 0; f < nf; ++f) {
+            int64_t a = (int64_t)hits[u * nf + f];
+            int64_t b = (int64_t)universe_hits[f] - a;
+            int64_t c = (int64_t)user_sizes[u] - a;
+            int64_t d = (int64_t)universe_size - a - b - c;
+            out[u][f] = ContingencyCounts{a, b, c, d};
+        }
+    return out;
+}
+}  // namespace
+
 std::vector<std::vector<ContingencyCounts>> lola_contingency(const Igd& igd, const std::vector<const RegionSet*>& user_sets,
                                                              const RegionSet& universe, int32_t min_overlap) {
     if (igd.num_files() == 0) throw Error("Database is empty");       // LolaError::EmptyDatabase, enrichment.rs:189-191
     if (universe.regions.empty()) throw Error("Universe is empty");   // LolaError::EmptyUniverse, enrichment.rs:194-196
     std::vector<const RegionSet*> all(user_sets);
     all.push_back(&universe);
-    const size_t nf = igd.num_files();
     std::vector<uint64_t> hits = igd.count_region_hits_batch(all, min_overlap, false);  // one device pass
-    const uint64_t* universe_hits = hits.data() + user_sets.size() * nf;
-    std::vector<std::vector<ContingencyCounts>> out(user_sets.size(), std::vector<ContingencyCounts>(nf));
-    for (size_t u = 0; u < user_sets.size(); ++u)
-        for (size_t f = 0; f < nf; ++f) {
-            int64_t a = (int64_t)hits[u * nf + f];
-            int64_t b = (int64_t)universe_hits[f] - a;
-            int64_t c = (int64_t)user_sets[u]->regions.size() - a;
-            int64_t d = (int64_t)universe.regions.size() - a - b - c;
-            out[u][f] = ContingencyCounts{a, b, c, d};
-        }
-    return out;
+    std::vector<uint64_t> user_sizes(user_sets.size());
+    for (size_t u = 0; u < user_sets.size(); ++u) user_sizes[u] = user_sets[u]->regions.size();
+    return contingency_tables(hits, igd.num_files(), user_sizes, universe.regions.size());
+}
+
+std::vector<std::vector<ContingencyCounts>> lola_contingency_bed_files(const Igd& igd, const std::vector<std::string>& user_paths,
+                                                                       const std::string& universe_path, int32_t min_overlap) {
+    if (igd.num_files() == 0) throw Error("Database is empty");  // LolaError::EmptyDatabase; an empty universe fails in the parse
+    std::vector<std::string> all(user_paths);
+    all.push_back(universe_path);
+    Igd::BedCounts h = igd.count_bed_files(all, min_overlap, false);  // one device pass
+    const uint64_t universe_size = h.set_regions.back();
+    h.set_regions.pop_back();
+    return contingency_tables(h.matrix, igd.num_files(), h.set_regions, universe_size);
 }
 
 }  // namespace gtars

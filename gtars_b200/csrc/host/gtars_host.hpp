@@ -269,6 +269,13 @@ class Igd {
     // inflated by zlib) and the texts go back to back.  Chromosome ids follow the names' first appearance in the files.  Errors
     // name the file's path.
     static std::unique_ptr<Igd> from_bed_files(std::shared_ptr<Device> dev, const std::vector<std::string>& paths);
+    // count_region_hits_batch (pairwise: count_set_overlaps) of query sets given as BED files, each parsed on the device
+    // (gtgpu_igd_count_bed; the gzip form when every path ends in ".gz", as from_bed_files).  matrix: [paths x n_files];
+    // set_regions: every file's region lines (RegionSet::len).  Errors name the file's path.  A database Igd only.
+    struct BedCounts {
+        std::vector<uint64_t> matrix, set_regions;
+    };
+    BedCounts count_bed_files(const std::vector<std::string>& paths, int32_t min_overlap, bool pairwise) const;
     // gtgpu_igd_info: n_files, records kept, device bytes, LUT shift (a database Igd only)
     std::array<uint64_t, 4> info() const;
 
@@ -293,5 +300,9 @@ class Igd {
 // run_lola up to the contingency tables (enrichment.rs:198-220): [user set][db set].  Fisher / ranking stay with the caller.
 std::vector<std::vector<ContingencyCounts>> lola_contingency(const Igd& igd, const std::vector<const RegionSet*>& user_sets,
                                                              const RegionSet& universe, int32_t min_overlap = 1);
+// lola_contingency([RegionSet(p) for p in user_paths], RegionSet(universe_path)) with every file parsed on the device, the
+// universe counted as the last set of the same pass (Igd::count_bed_files).
+std::vector<std::vector<ContingencyCounts>> lola_contingency_bed_files(const Igd& igd, const std::vector<std::string>& user_paths,
+                                                                       const std::string& universe_path, int32_t min_overlap = 1);
 
 }  // namespace gtars

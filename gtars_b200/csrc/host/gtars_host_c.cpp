@@ -335,5 +335,28 @@ int gth_lola_contingency(void* g, uint64_t n_user, void** user_sets, void* unive
         return 0;
     }, 1);
 }
+// out: [n_paths x num_files] u64, out_set_regions: n_paths u64
+int gth_igd_count_bed_files(void* g, uint64_t n_paths, const char** paths, int32_t min_overlap, int pairwise, uint64_t* out,
+                            uint64_t* out_set_regions) {
+    return guard([&]() -> int {
+        auto r = ((Igd*)g)->count_bed_files(std::vector<std::string>(paths, paths + n_paths), min_overlap, pairwise != 0);
+        std::copy(r.matrix.begin(), r.matrix.end(), out);
+        std::copy(r.set_regions.begin(), r.set_regions.end(), out_set_regions);
+        return 0;
+    }, 1);
+}
+int gth_lola_contingency_bed_files(void* g, uint64_t n_user, const char** user_paths, const char* universe_path, int32_t min_overlap,
+                                   int64_t* out) {
+    return guard([&]() -> int {
+        auto t = lola_contingency_bed_files(*(Igd*)g, std::vector<std::string>(user_paths, user_paths + n_user), universe_path,
+                                            min_overlap);
+        size_t k = 0;
+        for (auto& row : t)
+            for (auto& c : row) {
+                out[k++] = c.a; out[k++] = c.b; out[k++] = c.c; out[k++] = c.d;
+            }
+        return 0;
+    }, 1);
+}
 
 }  // extern "C"

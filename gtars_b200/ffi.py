@@ -77,6 +77,8 @@ SIGNATURES = {
     "gtgpu_igd_count_set_overlaps": (_i32, [_vp, _u64, _vp, _vp, _vp, _vp, _i32, _vp]),
     "gtgpu_igd_count_region_hits": (_i32, [_vp, _u64, _vp, _vp, _vp, _vp, _i32, _vp]),
     "gtgpu_igd_count_dev": (_i32, [_vp, _i32, _u64, _vp, _vp, _vp, _vp, _i32, _vp]),
+    "gtgpu_igd_count_bed": (_i32, [_vp, _i32, _u64, _vp, _vp, _u32, _vp, _vp, _i32, _vp, _vp]),
+    "gtgpu_igd_count_bed_gz": (_i32, [_vp, _i32, _u64, _vp, _u64, _vp, _vp, _u32, _vp, _vp, _i32, _vp, _vp]),
     "gtgpu_comm_unique_id": (_i32, [_vp]),
     "gtgpu_comm_init": (_i32, [_vp, _i32, _i32, _vp]),
     "gtgpu_comm_free": (_i32, [_vp]),
@@ -616,6 +618,30 @@ class Igd:
 
     def count_region_hits(self, set_offsets, chr, start, end, min_overlap=1):
         return self._count(lib().gtgpu_igd_count_region_hits, set_offsets, chr, start, end, min_overlap)
+
+    def _count_bed(self, n_sets, chrom_names, call):
+        blob, offs = _names_blob(chrom_names)
+        out = np.zeros((n_sets, self.n_files), dtype=np.uint64)
+        regions = np.zeros(n_sets, dtype=np.uint64)
+        check(call(len(chrom_names), blob, _p(offs), _p(out), _p(regions)))
+        return out, regions
+
+    def count_bed_text(self, binary, text, file_offsets, chrom_names, min_overlap=1):
+        """gtgpu_igd_count_bed: count_region_hits (binary) / count_set_overlaps of query set s = text[file_offsets[s]:file_offsets[s
+        + 1]], parsed on the device; chrom_names[i] is the database's chromosome i.  Returns (uint64 [n_sets, n_files], the
+        sets' region lines).  `text` may be a uint8 numpy array."""
+        fo = _arr(file_offsets, np.uint64)
+        n = len(fo) - 1
+        return self._count_bed(n, chrom_names, lambda nn, blob, offs, out, reg: lib().gtgpu_igd_count_bed(
+            self._h, 1 if binary else 0, n, _text_ptr(text), _p(fo), nn, blob, offs, min_overlap, out, reg))
+
+    def count_bed_gz(self, binary, gz, file_members, member_offsets, chrom_names, min_overlap=1):
+        """gtgpu_igd_count_bed_gz: query set s = gzip members [file_members[s], file_members[s + 1]) of `gz`, inflated and parsed on
+        the device.  Returns (matrix, the sets' region lines) as count_bed_text does."""
+        fm, mo = _arr(file_members, np.uint64), _arr(member_offsets, np.uint64)
+        n = len(fm) - 1
+        return self._count_bed(n, chrom_names, lambda nn, blob, offs, out, reg: lib().gtgpu_igd_count_bed_gz(
+            self._h, 1 if binary else 0, n, _p(fm), len(mo) - 1, _text_ptr(gz), _p(mo), nn, blob, offs, min_overlap, out, reg))
 
     def count_sharded(self, binary, n_files_global, set_offsets, chr, start, end, min_overlap=1, out=None):
         """`out` (optional): a caller-owned uint64 [n_sets, n_files_global] array, e.g. pinned memory from pinned_empty."""

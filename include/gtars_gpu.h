@@ -378,6 +378,22 @@ int32_t gtgpu_igd_count_region_hits(gtgpu_igd* igd, uint64_t n_sets, const uint6
 /* device-resident core: d_set_of[i] = set index of query i; d_out ([n_sets x n_files] u64) is accumulated into */
 int32_t gtgpu_igd_count_dev(gtgpu_igd* igd, int32_t binary, uint64_t n, const uint32_t* d_set_of, const uint32_t* d_chr,
                             const uint32_t* d_start, const uint32_t* d_end, int32_t min_overlap, uint64_t* d_out);
+/* Igd::count_region_hits (binary = 1) / Igd::count_set_overlaps (binary = 0) for n_sets query sets given as BED files, parsed on
+ * the device: set s = text[file_offsets[s], file_offsets[s+1]) (any total size), or the gzip members [file_members[s],
+ * file_members[s+1]) of gz / member_offsets (as in gtgpu_igd_build_bed_gz).  Line rules, windows, the header rule per file and
+ * the errors ("file k, line j"; "file k: ... 0 regions found"; at most 262 144 distinct names and fewer than 2^32 - 1 region
+ * lines, else GTGPU_ERR_UNSUPPORTED) are those of gtgpu_igd_build_bed.  Chromosome names map through the caller's table (the
+ * database's names, as gtgpu_igd_build_bed returns them or as the caller of gtgpu_igd_build numbered them), looked up as
+ * gtgpu_parse_bed does; a name not in it contributes no hits.  out = [n_sets x n_files] u64 row-major (caller-allocated,
+ * overwritten); out_set_regions[s] = the region lines of set s (RegionSet::len: every region line, unknown names and start >= end
+ * included: the |user set| / |universe| of run_lola's tables).  min_overlap >= 1.  On a multi-device ctx the parse runs on the
+ * first device and every device reads the parsed queries from there. */
+int32_t gtgpu_igd_count_bed(gtgpu_igd* igd, int32_t binary, uint64_t n_sets, const char* text, const uint64_t* file_offsets,
+                            uint32_t n_names, const char* names, const uint32_t* name_offsets, int32_t min_overlap,
+                            uint64_t* out, uint64_t* out_set_regions);
+int32_t gtgpu_igd_count_bed_gz(gtgpu_igd* igd, int32_t binary, uint64_t n_sets, const uint64_t* file_members, uint64_t n_members,
+                               const uint8_t* gz, const uint64_t* member_offsets, uint32_t n_names, const char* names,
+                               const uint32_t* name_offsets, int32_t min_overlap, uint64_t* out, uint64_t* out_set_regions);
 
 /* ---- multi-GPU: the LOLA database sharded by region set, one ncclAllGather (run_lola's count matrices,
  * gtars-lola/src/enrichment.rs:198-211) ------------------------------------------------------------------------------
