@@ -134,6 +134,10 @@ extern "C" {
                                   member_offsets: *const u64, out_n_chroms: *mut u32, out_chrom_names: *mut *mut gtgpu_buf,
                                   out_chrom_name_offsets: *mut *mut gtgpu_buf, out_igd: *mut *mut gtgpu_igd) -> i32;
     pub fn gtgpu_igd_free(igd: *mut gtgpu_igd) -> i32;
+    /// Igd::save of a database built any way: the .igd file's bytes (u8 buffer), and per file the .tsv region count and width
+    /// sum (n_files each).  names: the chromosome names by id (n_names + 1 u32 offsets), n_names == the igd's chromosome count.
+    pub fn gtgpu_igd_serialize(igd: *mut gtgpu_igd, n_names: u32, names: *const u8, name_offsets: *const u32,
+                               out_igd_bytes: *mut *mut gtgpu_buf, out_file_regions: *mut u64, out_file_width_sums: *mut u64) -> i32;
     pub fn gtgpu_igd_info(igd: *const gtgpu_igd, info: *mut u64) -> i32;
     pub fn gtgpu_igd_count_set_overlaps(igd: *mut gtgpu_igd, n_sets: u64, set_offsets: *const u64, chr: *const u32,
                                         start: *const u32, end: *const u32, min_overlap: i32, out: *mut u64) -> i32;

@@ -60,7 +60,8 @@ def lib():
             "gth_gtok_read": (vp, [cp]),
             "gth_igd_single": (vp, [vp, vp]), "gth_igd_find_pairs": (vp, [vp, vp, i32]),
             "gth_igd_count_per_query": (vp, [vp, vp, i32]),
-            "gth_igd_save_sets": (C.c_int, [u64, vp, vp, cp]), "gth_igd_from_file": (vp, [vp, cp]),
+            "gth_igd_save_sets": (C.c_int, [u64, vp, vp, cp]), "gth_igd_save": (C.c_int, [vp, u64, vp, cp]),
+            "gth_igd_from_file": (vp, [vp, cp]),
             "gth_igd_from_bed_files": (vp, [vp, u64, vp]), "gth_igd_info": (C.c_int, [vp, vp]),
             "gth_igd_new": (vp, [vp, u64, vp]), "gth_igd_free": (None, [vp]), "gth_igd_num_files": (u64, [vp]),
             "gth_igd_count": (C.c_int, [vp, u64, vp, i32, C.c_int, vp]),
@@ -467,11 +468,12 @@ class Igd:
             self._h = None
 
     def save(self, path, names=None):
-        """Igd::save (igd.rs:418-486): `path` (.igd) plus the companion .tsv, byte-for-byte the reference's files."""
-        names = list(names) if names is not None else [f"set{i}" for i in range(len(self._sets))]
-        arr = (C.c_void_p * max(len(self._sets), 1))(*[s._h for s in self._sets])
+        """Igd::save (igd.rs:418-486): `path` (.igd) plus the companion .tsv, byte-for-byte the reference's files, written from
+        the database on the device (gtgpu_igd_serialize) however it was built.  names[f] names file f in the .tsv (default
+        set{f}).  A from_single_region_set Igd has no database to save and raises GtarsError."""
+        names = list(names) if names is not None else [f"set{i}" for i in range(self.num_files())]
         nm = (C.c_char_p * max(len(names), 1))(*[n.encode() for n in names])
-        if lib().gth_igd_save_sets(len(self._sets), arr, nm, os.fsencode(path)):
+        if lib().gth_igd_save(self._h, len(names), nm, os.fsencode(path)):
             _fail()
 
     @classmethod

@@ -242,6 +242,15 @@ struct gtgpu_igd {
     std::vector<void*> allocs;
     uint64_t device_bytes = 0;
     std::vector<gtgpu_igd*> shards;
+    // What gtgpu_igd_serialize needs beyond the records.  Per file: the input's region lines with start < end (as u32) and the
+    // wrapping sum of their int32 widths (the .tsv).  Per chromosome: its largest kept end (the contig's tile count), and
+    // h_first: the smallest input index of a kept record on it or, when contig_by_file, the smallest file with one (the rank
+    // of the contig in the reference's creation order; UINT32_MAX: none).  A shard's values count from its own first file /
+    // record (file0 / rec0 in the group's input).
+    std::vector<uint64_t> h_file_regions, h_file_widths;
+    std::vector<uint32_t> h_first, h_max_end;
+    bool contig_by_file = false;
+    uint64_t file0 = 0, rec0 = 0;
 };
 
 namespace gtgpu {

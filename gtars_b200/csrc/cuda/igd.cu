@@ -81,6 +81,62 @@ __global__ void igd_chrom_keys_kernel(uint64_t n, uint32_t n_chroms, const uint3
     }
 }
 
+// The .tsv statistics of every input file (Igd::from_named_region_sets, igd.rs:285-317): the region lines with start < end as
+// u32 (dropped negative ones included) and the wrapping u64 sum of their widths (i32 end - i32 start, widened).  A file's records
+// are contiguous, so a warp whose lanes share one file adds its sums once.
+__global__ void igd_file_stats_kernel(uint64_t n, const uint32_t* __restrict__ start, const uint32_t* __restrict__ end,
+                                      const uint32_t* __restrict__ file, unsigned long long* __restrict__ regions,
+                                      unsigned long long* __restrict__ widths) {
+    constexpr uint32_t FULL = 0xFFFFFFFFu;
+    const uint32_t lane = threadIdx.x & 31;
+    const uint64_t stride = (uint64_t)gridDim.x * blockDim.x;
+    for (uint64_t base = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x - lane; base < n; base += stride) {
+        const uint64_t i = base + lane;
+        const bool ok = i < n;
+        const uint32_t s = ok ? start[i] : 0, e = ok ? end[i] : 0, f = ok ? file[i] : 0;
+        const bool region = ok && s < e;
+        unsigned long long c = region, w = region ? (unsigned long long)(long long)(int32_t)(e - s) : 0ull;
+        const uint32_t f0 = __shfl_sync(FULL, f, 0);  // lane 0 is always in range
+        if (__all_sync(FULL, !ok || f == f0)) {
+#pragma unroll
+            for (int o = 16; o; o >>= 1) {
+                c += __shfl_xor_sync(FULL, c, o);
+                w += __shfl_xor_sync(FULL, w, o);
+            }
+            if (lane == 0 && c) {
+                atomicAdd(regions + f0, c);
+                atomicAdd(widths + f0, w);
+            }
+        } else if (region) {
+            atomicAdd(regions + f, 1ull);
+            atomicAdd(widths + f, w);
+        }
+    }
+}
+
+// first[c] = min over the kept records of chromosome c of their input index (file == nullptr) or their file.  chrkey is
+// sorted, so a warp mostly holds one chromosome and reduces before its one atomic.
+__global__ void igd_first_kept_kernel(uint64_t n, const uint32_t* __restrict__ chrkey, const uint32_t* __restrict__ perm,
+                                      const uint32_t* __restrict__ file, uint32_t* __restrict__ first) {
+    constexpr uint32_t FULL = 0xFFFFFFFFu;
+    const uint32_t lane = threadIdx.x & 31;
+    const uint64_t stride = (uint64_t)gridDim.x * blockDim.x;
+    for (uint64_t base = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x - lane; base < n; base += stride) {
+        const uint64_t k = base + lane;
+        const bool ok = k < n;
+        const uint32_t c = ok ? chrkey[k] : 0;
+        uint32_t v = 0xFFFFFFFFu;
+        if (ok) v = file ? file[perm[k]] : perm[k];
+        const uint32_t c0 = __shfl_sync(FULL, c, 0);
+        if (__all_sync(FULL, !ok || c == c0)) {
+            v = __reduce_min_sync(FULL, v);
+            if (lane == 0) atomicMin(first + c0, v);
+        } else if (ok) {
+            atomicMin(first + c, v);
+        }
+    }
+}
+
 // packed[k] = segment << 32 | value: the running maximum of the low word inside a segment is a plain 64-bit max-scan
 __global__ void igd_pack_pmax_kernel(uint64_t n, const uint32_t* __restrict__ chrkey, const int32_t* __restrict__ end,
                                      unsigned long long* __restrict__ packed) {
@@ -303,13 +359,16 @@ using namespace gtgpu;
 
 // Multi-device group: the database is sharded by region set (run_lola's database axis, enrichment.rs:198-211): device r
 // builds its own record pool over sets [r * C, min((r + 1) * C, n_files)), C = ceil(n_files / devices), all in parallel.
+// contig_by_file: the records come from BED files, whose RegionSets the reference sorts by (name, start) before Igd::add sees them
+// (gtgpu_igd_serialize's contig order).
 static int32_t igd_build_one(gtgpu_ctx* ctx, uint64_t n_files, const uint64_t* file_offsets, uint32_t n_chroms, const uint32_t* chr,
-                             const uint32_t* start, const uint32_t* end, gtgpu_igd** out_igd);
+                             const uint32_t* start, const uint32_t* end, bool contig_by_file, gtgpu_igd** out_igd);
 static int32_t igd_build_dev(gtgpu_ctx* ctx, uint64_t n_files, uint32_t n_chroms, uint64_t total, const uint32_t* t_chr,
-                             const uint32_t* t_start, const uint32_t* t_end, const uint32_t* t_file, gtgpu_igd** out_igd);
+                             const uint32_t* t_start, const uint32_t* t_end, const uint32_t* t_file, bool contig_by_file,
+                             gtgpu_igd** out_igd);
 
 static int32_t igd_build_group(gtgpu_ctx* ctx, uint64_t n_files, const uint64_t* file_offsets, uint32_t n_chroms, const uint32_t* chr,
-                               const uint32_t* start, const uint32_t* end, gtgpu_igd** out_igd) {
+                               const uint32_t* start, const uint32_t* end, bool contig_by_file, gtgpu_igd** out_igd) {
     std::lock_guard<std::mutex> glk(ctx->group_mu);
     const size_t D = ctx->peers.size();
     const uint64_t cols = (n_files + D - 1) / D;
@@ -324,8 +383,13 @@ static int32_t igd_build_group(gtgpu_ctx* ctx, uint64_t n_files, const uint64_t*
         for (uint64_t f = lo; f <= hi; ++f) fo[f - lo] = file_offsets[f] - file_offsets[lo];
         const uint64_t r0 = file_offsets[lo];
         // (peers[0] is the group context itself: the single-device builder is called directly, not through the entry point)
-        return igd_build_one(ctx->peers[r], hi - lo, fo.data(), n_chroms, chr ? chr + r0 : nullptr, start ? start + r0 : nullptr,
-                             end ? end + r0 : nullptr, &g->shards[r]);
+        const int32_t st = igd_build_one(ctx->peers[r], hi - lo, fo.data(), n_chroms, chr ? chr + r0 : nullptr,
+                                         start ? start + r0 : nullptr, end ? end + r0 : nullptr, contig_by_file, &g->shards[r]);
+        if (st == GTGPU_OK) {
+            g->shards[r]->file0 = lo;
+            g->shards[r]->rec0 = r0;
+        }
+        return st;
     });
     if (s != GTGPU_OK) {
         const std::string msg = gtgpu_last_error();
@@ -337,6 +401,7 @@ static int32_t igd_build_group(gtgpu_ctx* ctx, uint64_t n_files, const uint64_t*
         g->device_bytes += sh->device_bytes;
     }
     g->shift = g->shards[0]->shift;
+    g->contig_by_file = contig_by_file;
     *out_igd = g.release();
     return GTGPU_OK;
 }
@@ -351,8 +416,8 @@ extern "C" int32_t gtgpu_igd_build(gtgpu_ctx* ctx, uint64_t n_files, const uint6
     if (total && (!chr || !start || !end)) return fail(GTGPU_ERR_INVALID, "igd_build: null record arrays");
     if (total >= 0xFFFFFFFFull || n_files >= 0xFFFFFFFFull || n_chroms >= 0x7FFFFFFFu)
         return fail(GTGPU_ERR_UNSUPPORTED, "igd_build: too many records");
-    if (ctx->peers.size() > 1) return igd_build_group(ctx, n_files, file_offsets, n_chroms, chr, start, end, out_igd);
-    return igd_build_one(ctx, n_files, file_offsets, n_chroms, chr, start, end, out_igd);
+    if (ctx->peers.size() > 1) return igd_build_group(ctx, n_files, file_offsets, n_chroms, chr, start, end, false, out_igd);
+    return igd_build_one(ctx, n_files, file_offsets, n_chroms, chr, start, end, false, out_igd);
 } GT_CATCH
 
 // ---- a database from its BED files' text, parsed on the device --------------------------------------------------------------
@@ -364,12 +429,12 @@ static int32_t igd_build_parsed(gtgpu_ctx* ctx, uint64_t n_files, BedFilesRecord
     const uint32_t n_chroms = r.n_names;
     gtgpu_igd* g = nullptr;
     if (ctx->peers.size() > 1) {
-        GT_TRY(igd_build_group(ctx, n_files, r.file_offsets.data(), n_chroms, r.chr.u32(), r.start.u32(), r.end.u32(), &g));
+        GT_TRY(igd_build_group(ctx, n_files, r.file_offsets.data(), n_chroms, r.chr.u32(), r.start.u32(), r.end.u32(), true, &g));
         GT_CUDA(cudaSetDevice(ctx->device));  // the parsed records are freed on their device
     } else {
         std::lock_guard<std::mutex> lk(ctx->mu);
         GT_CUDA(cudaSetDevice(ctx->device));
-        GT_TRY(igd_build_dev(ctx, n_files, n_chroms, r.n, r.chr.u32(), r.start.u32(), r.end.u32(), r.file.u32(), &g));
+        GT_TRY(igd_build_dev(ctx, n_files, n_chroms, r.n, r.chr.u32(), r.start.u32(), r.end.u32(), r.file.u32(), true, &g));
     }
     *out_n_chroms = n_chroms;
     *out_names = r.names.release();
@@ -447,23 +512,25 @@ static int32_t igd_records_to_device(gtgpu_ctx* ctx, TempPool& tp, uint64_t n_fi
 }
 
 static int32_t igd_build_one(gtgpu_ctx* ctx, uint64_t n_files, const uint64_t* file_offsets, uint32_t n_chroms, const uint32_t* chr,
-                             const uint32_t* start, const uint32_t* end, gtgpu_igd** out_igd) {
+                             const uint32_t* start, const uint32_t* end, bool contig_by_file, gtgpu_igd** out_igd) {
     std::lock_guard<std::mutex> lk(ctx->mu);
     GT_CUDA(cudaSetDevice(ctx->device));
     TempPool tp;
     uint32_t *t_chr, *t_start, *t_end, *t_file;
     GT_TRY(igd_records_to_device(ctx, tp, n_files, file_offsets, chr, start, end, &t_chr, &t_start, &t_end, &t_file));
-    return igd_build_dev(ctx, n_files, n_chroms, file_offsets[n_files], t_chr, t_start, t_end, t_file, out_igd);
+    return igd_build_dev(ctx, n_files, n_chroms, file_offsets[n_files], t_chr, t_start, t_end, t_file, contig_by_file, out_igd);
 }
 
 // The build from device-resident records of this ctx's device (record i belongs to file t_file[i]).  The caller holds ctx->mu.
 static int32_t igd_build_dev(gtgpu_ctx* ctx, uint64_t n_files, uint32_t n_chroms, uint64_t total, const uint32_t* t_chr,
-                             const uint32_t* t_start, const uint32_t* t_end, const uint32_t* t_file, gtgpu_igd** out_igd) {
+                             const uint32_t* t_start, const uint32_t* t_end, const uint32_t* t_file, bool contig_by_file,
+                             gtgpu_igd** out_igd) {
     cudaStream_t st = ctx->stream;
     gtgpu_igd* g = new gtgpu_igd();
     g->ctx = ctx;
     g->n_files = n_files;
     g->n_chroms = n_chroms;
+    g->contig_by_file = contig_by_file;
     struct Guard {  // a failed build frees what it allocated
         gtgpu_igd* g;
         ~Guard() { if (g) gtgpu_igd_free(g); }
@@ -493,6 +560,35 @@ static int32_t igd_build_dev(gtgpu_ctx* ctx, uint64_t n_files, uint32_t n_chroms
     const uint64_t n_rec = g->h_off[n_chroms];
     g->n_records = n_rec;
 
+    // ---- what a save needs besides the records: the .tsv statistics of every file, the first kept record of every chromosome
+    {
+        unsigned long long* d_stats;
+        uint32_t* d_first;
+        GT_TRY(tp.get(2 * n_files, &d_stats));
+        GT_TRY(tp.get(n_chroms, &d_first));
+        if (n_files) GT_CUDA(cudaMemsetAsync(d_stats, 0, 2 * n_files * 8, st));
+        if (n_chroms) GT_CUDA(cudaMemsetAsync(d_first, 0xFF, (uint64_t)n_chroms * 4, st));
+        if (total) {
+            igd_file_stats_kernel<<<grid_for(ctx, total), 256, 0, st>>>(total, t_start, t_end, t_file, d_stats, d_stats + n_files);
+            ctx->launches++;
+        }
+        if (n_rec) {
+            igd_first_kept_kernel<<<grid_for(ctx, n_rec), 256, 0, st>>>(n_rec, pooled.key, pooled.perm, contig_by_file ? t_file : nullptr,
+                                                                        d_first);
+            ctx->launches++;
+        }
+        GT_CUDA(cudaGetLastError());
+        g->h_file_regions.assign(n_files, 0);
+        g->h_file_widths.assign(n_files, 0);
+        g->h_first.assign(n_chroms, 0xFFFFFFFFu);
+        if (n_files) {
+            GT_CUDA(cudaMemcpyAsync(g->h_file_regions.data(), d_stats, n_files * 8, cudaMemcpyDeviceToHost, st));
+            GT_CUDA(cudaMemcpyAsync(g->h_file_widths.data(), d_stats + n_files, n_files * 8, cudaMemcpyDeviceToHost, st));
+        }
+        if (n_chroms) GT_CUDA(cudaMemcpyAsync(g->h_first.data(), d_first, (uint64_t)n_chroms * 4, cudaMemcpyDeviceToHost, st));
+        GT_CUDA(cudaStreamSynchronize(st));
+    }
+
     // ---- 2. the kept records in pooled order, running max of ends per chromosome ------------------------------------
     GT_TRY(dev_alloc(g, n_rec, &g->d_start));
     GT_TRY(dev_alloc(g, n_rec, &g->d_end));
@@ -521,6 +617,7 @@ static int32_t igd_build_dev(gtgpu_ctx* ctx, uint64_t n_files, uint32_t n_chroms
         }
         GT_CUDA(cudaStreamSynchronize(st));
     }
+    g->h_max_end = last_pmax;
 
     // ---- 3. bin LUTs over starts and running maxima: at most ~8 M bins per family --------------------------------------
     uint32_t shift = 0;
@@ -863,4 +960,247 @@ extern "C" int32_t gtgpu_igd_count_bed_gz(gtgpu_igd* igd, int32_t binary, uint64
                                         "igd_count_bed_gz", &r));
     }
     return igd_count_parsed(igd, binary != 0, n_sets, r, min_overlap, out, out_set_regions);
+} GT_CATCH
+
+// ---- .igd bytes of a database, written from the device -----------------------------------------------------------------------
+// Igd::save (igd.rs:418-486) after from_named_region_sets: a kept record sits in every 16 384-bp tile from start / nbp to
+// (end - 1) / nbp of its contig, a tile holds its records stable-sorted by start with ties in (file, insertion) order, and the
+// contigs come in the order Igd::add created them.  The pooled order (chromosome, start, file, insertion) filtered to one tile
+// is that tile's order, so the records are expanded to one entry per tile they reach and sorted stably by (contig rank, tile).
+namespace gtgpu {
+
+constexpr int32_t IGD_NBP = 16384;  // igd.rs:14
+
+// tiles[k] = the tiles record k reaches; tiles[n] = 0 closes the scan
+__global__ void igd_tile_counts_kernel(uint64_t n, const int32_t* __restrict__ start, const int32_t* __restrict__ end,
+                                       unsigned long long* __restrict__ tiles) {
+    const uint64_t stride = (uint64_t)gridDim.x * blockDim.x;
+    for (uint64_t k = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x; k <= n; k += stride)
+        tiles[k] = k < n ? (unsigned long long)((end[k] - 1) / IGD_NBP - start[k] / IGD_NBP + 1) : 0ull;
+}
+
+// one (global tile, record) pair per tile entry at the record's scanned offset; global tile = its contig's first tile + tile
+__global__ void igd_expand_tiles_kernel(uint64_t n, const int32_t* __restrict__ start, const int32_t* __restrict__ end,
+                                        const uint32_t* __restrict__ chr, const uint32_t* __restrict__ tile_base,
+                                        const unsigned long long* __restrict__ offset, uint32_t* __restrict__ key,
+                                        uint32_t* __restrict__ rec) {
+    const uint64_t stride = (uint64_t)gridDim.x * blockDim.x;
+    for (uint64_t k = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x; k < n; k += stride) {
+        const int32_t t0 = start[k] / IGD_NBP, t1 = (end[k] - 1) / IGD_NBP;
+        const uint32_t b = tile_base[chr[k]] + (uint32_t)t0;
+        const uint64_t o = offset[k];
+        for (int32_t t = 0; t <= t1 - t0; ++t) {
+            key[o + t] = b + (uint32_t)t;
+            rec[o + t] = (uint32_t)k;
+        }
+    }
+}
+
+// entry j of the sorted order as the file's 16-byte record (file_idx, start, end, value = 0), one 16-byte store
+__global__ void igd_format_records_kernel(uint64_t n, const uint32_t* __restrict__ perm, const uint32_t* __restrict__ rec,
+                                          const uint32_t* __restrict__ file, const int32_t* __restrict__ start,
+                                          const int32_t* __restrict__ end, int4* __restrict__ out) {
+    const uint64_t stride = (uint64_t)gridDim.x * blockDim.x;
+    for (uint64_t j = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x; j < n; j += stride) {
+        const uint32_t k = rec[perm[j]];
+        out[j] = make_int4((int32_t)file[k], start[k], end[k], 0);
+    }
+}
+
+__global__ void igd_add_u32_kernel(uint64_t n, uint32_t* __restrict__ v, uint32_t add) {
+    const uint64_t stride = (uint64_t)gridDim.x * blockDim.x;
+    for (uint64_t k = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x; k < n; k += stride) v[k] += add;
+}
+
+}  // namespace gtgpu
+
+// The records of a group igd on ctx's device in pooled order: every shard's arrays copied over (cudaMemcpyAsync, any device),
+// file indexes rebased by the shard's first file, then stably sorted by (chromosome, start) as igd_build_dev step 1 does; shard
+// order is file order, so ties keep (file, insertion).  The caller holds ctx->group_mu and ctx->mu.
+static int32_t igd_gather_shards(gtgpu_igd* g, TempPool& tp, int32_t** out_start, int32_t** out_end, uint32_t** out_file,
+                                 uint32_t** out_chr) {
+    gtgpu_ctx* ctx = g->ctx;
+    cudaStream_t st = ctx->stream;
+    const uint64_t n = g->n_records;
+    const uint32_t n_chroms = g->n_chroms;
+    uint32_t *c_start, *c_end, *c_file, *c_chr;
+    uint64_t* d_off64;
+    GT_TRY(tp.get(n, &c_start));
+    GT_TRY(tp.get(n, &c_end));
+    GT_TRY(tp.get(n, &c_file));
+    GT_TRY(tp.get(n, &c_chr));
+    GT_TRY(tp.get(n, (uint32_t**)out_start));
+    GT_TRY(tp.get(n, (uint32_t**)out_end));
+    GT_TRY(tp.get(n, out_file));
+    GT_TRY(tp.get(n, out_chr));
+    GT_TRY(tp.get((uint64_t)n_chroms + 1, &d_off64));
+    std::vector<uint64_t> off64(n_chroms + 1);
+    uint64_t base = 0;
+    for (gtgpu_igd* sh : g->shards) {
+        const uint64_t m = sh->n_records;
+        if (m == 0) continue;
+        GT_CUDA(cudaMemcpyAsync(c_start + base, sh->d_start, m * 4, cudaMemcpyDefault, st));
+        GT_CUDA(cudaMemcpyAsync(c_end + base, sh->d_end, m * 4, cudaMemcpyDefault, st));
+        GT_CUDA(cudaMemcpyAsync(c_file + base, sh->d_file, m * 4, cudaMemcpyDefault, st));
+        igd_add_u32_kernel<<<grid_for(ctx, m), 256, 0, st>>>(m, c_file + base, (uint32_t)sh->file0);
+        for (uint32_t c = 0; c <= n_chroms; ++c) off64[c] = base + sh->h_off[c];
+        GT_CUDA(cudaMemcpyAsync(d_off64, off64.data(), off64.size() * 8, cudaMemcpyHostToDevice, st));
+        GT_TRY(launch_fill_set_ids(ctx, n_chroms, d_off64, c_chr));
+        ctx->launches++;
+        GT_CUDA(cudaGetLastError());
+        GT_CUDA(cudaStreamSynchronize(st));  // off64 is reused for the next shard
+        base += m;
+    }
+    if (n == 0) return GTGPU_OK;
+    PermSorter pooled;
+    GT_TRY(pooled.init(ctx, n));
+    GT_TRY(pooled.pass(c_start, 0));
+    GT_TRY(pooled.pass(c_chr, bits_for_value(n_chroms)));
+    GT_TRY(launch_gather_u32(ctx, n, c_start, pooled.perm, (uint32_t*)*out_start));
+    GT_TRY(launch_gather_u32(ctx, n, c_end, pooled.perm, (uint32_t*)*out_end));
+    GT_TRY(launch_gather_u32(ctx, n, c_file, pooled.perm, *out_file));
+    GT_TRY(launch_gather_u32(ctx, n, c_chr, pooled.perm, *out_chr));
+    GT_CUDA(cudaStreamSynchronize(st));
+    return GTGPU_OK;
+}
+
+// n kept records in pooled order on ctx's device -> the record payload of the file (16 bytes per tile entry) at buf + header,
+// where the header is written from the tile counts.  tile_base[c]: the first global tile of chromosome c's contig; the contigs'
+// tiles are numbered in file order, n_tiles in all.  The caller holds ctx->mu.
+static int32_t igd_write_tiles_locked(gtgpu_ctx* ctx, TempPool& tp, uint64_t n, const int32_t* d_start, const int32_t* d_end,
+                                      const uint32_t* d_file, const uint32_t* d_chr, const std::vector<uint32_t>& tile_base,
+                                      uint64_t n_tiles, uint64_t header_bytes, BufPtr* out_buf, std::vector<uint32_t>* tile_off) {
+    cudaStream_t st = ctx->stream;
+    unsigned long long *d_tiles, *d_toff;
+    char* d_scan_tmp;
+    GT_TRY(tp.get(n + 1, &d_tiles));
+    GT_TRY(tp.get(n + 1, &d_toff));
+    GT_TRY(tp.get(exclusive_scan_temp_bytes(n + 1, 8), &d_scan_tmp));
+    igd_tile_counts_kernel<<<grid_for(ctx, n + 1), 256, 0, st>>>(n, d_start, d_end, d_tiles);
+    ctx->launches++;
+    GT_CUDA(cudaGetLastError());
+    GT_TRY(exclusive_scan<unsigned long long>(ctx, d_tiles, d_toff, n + 1, d_scan_tmp));
+    uint64_t entries = 0;
+    GT_CUDA(cudaMemcpyAsync(&entries, d_toff + n, 8, cudaMemcpyDeviceToHost, st));
+    GT_CUDA(cudaStreamSynchronize(st));
+    if (entries >= 0xFFFFFFFFull)
+        return fail(GTGPU_ERR_UNSUPPORTED, "igd_serialize: " + std::to_string(entries) + " tile entries (at most 2^32 - 2)");
+    uint32_t *d_key, *d_rec, *d_tile_base, *d_tile_off;
+    int4* d_payload;
+    GT_TRY(tp.get(entries, &d_key));
+    GT_TRY(tp.get(entries, &d_rec));
+    GT_TRY(tp.get(tile_base.size(), &d_tile_base));
+    GT_TRY(tp.get(n_tiles + 1, &d_tile_off));
+    GT_TRY(tp.get(entries, &d_payload));
+    if (!tile_base.empty())
+        GT_CUDA(cudaMemcpyAsync(d_tile_base, tile_base.data(), tile_base.size() * 4, cudaMemcpyHostToDevice, st));
+    BufPtr buf;
+    GT_TRY(buf_new(ctx, header_bytes + entries * 16, 1, &buf));
+    tile_off->assign(n_tiles + 1, 0);
+    if (entries) {
+        igd_expand_tiles_kernel<<<grid_for(ctx, n), 256, 0, st>>>(n, d_start, d_end, d_chr, d_tile_base, d_toff, d_key, d_rec);
+        ctx->launches++;
+        GT_CUDA(cudaGetLastError());
+        PermSorter by_tile;
+        GT_TRY(by_tile.init(ctx, entries));
+        GT_TRY(by_tile.pass(d_key, bits_for_value(n_tiles - 1)));
+        GT_TRY(launch_key_offsets(ctx, entries, by_tile.key, (uint32_t)n_tiles, d_tile_off));
+        igd_format_records_kernel<<<grid_for(ctx, entries), 256, 0, st>>>(entries, by_tile.perm, d_rec, d_file, d_start, d_end,
+                                                                           d_payload);
+        ctx->launches++;
+        GT_CUDA(cudaGetLastError());
+        GT_CUDA(cudaMemcpyAsync(tile_off->data(), d_tile_off, (n_tiles + 1) * 4, cudaMemcpyDeviceToHost, st));
+        GT_CUDA(cudaMemcpyAsync((char*)buf->block.ptr + header_bytes, d_payload, entries * 16, cudaMemcpyDeviceToHost, st));
+        GT_CUDA(cudaStreamSynchronize(st));  // by_tile is freed when it leaves
+    }
+    *out_buf = std::move(buf);
+    return GTGPU_OK;
+}
+
+extern "C" int32_t gtgpu_igd_serialize(gtgpu_igd* g, uint32_t n_names, const char* names, const uint32_t* name_offsets,
+                                       gtgpu_buf** out_igd_bytes, uint64_t* out_file_regions, uint64_t* out_file_width_sums) try {
+    if (!g || !out_igd_bytes || (g->n_files && (!out_file_regions || !out_file_width_sums)) || (n_names && (!names || !name_offsets)))
+        return fail(GTGPU_ERR_INVALID, "igd_serialize: null argument");
+    if (n_names != g->n_chroms)
+        return fail(GTGPU_ERR_INVALID, "igd_serialize: " + std::to_string(n_names) + " names for " + std::to_string(g->n_chroms) +
+                                           " chromosomes");
+    for (uint32_t c = 0; c < n_names; ++c)
+        if (name_offsets[c] > name_offsets[c + 1]) return fail(GTGPU_ERR_INVALID, "igd_serialize: name_offsets not monotone");
+    gtgpu_ctx* ctx = g->ctx;
+    const std::vector<gtgpu_igd*> parts = g->shards.empty() ? std::vector<gtgpu_igd*>{g} : g->shards;
+    const uint32_t n_chroms = g->n_chroms;
+    // the .tsv numbers, and per chromosome its rank key and largest end over the parts
+    std::vector<uint64_t> first(n_chroms, UINT64_MAX);
+    std::vector<uint32_t> max_end(n_chroms, 0);
+    for (const gtgpu_igd* p : parts) {
+        std::copy(p->h_file_regions.begin(), p->h_file_regions.end(), out_file_regions + p->file0);
+        std::copy(p->h_file_widths.begin(), p->h_file_widths.end(), out_file_width_sums + p->file0);
+        const uint64_t rebase = g->contig_by_file ? p->file0 : p->rec0;
+        for (uint32_t c = 0; c < n_chroms; ++c) {
+            if (p->h_off[c + 1] == p->h_off[c]) continue;
+            first[c] = std::min<uint64_t>(first[c], p->h_first[c] + rebase);
+            max_end[c] = std::max(max_end[c], p->h_max_end[c]);
+        }
+    }
+    // contigs in creation order: by first kept input index (distinct), or for BED files by (first file, name bytes)
+    std::vector<uint32_t> order;
+    for (uint32_t c = 0; c < n_chroms; ++c)
+        if (first[c] != UINT64_MAX) order.push_back(c);
+    auto name = [&](uint32_t c) { return std::string(names + name_offsets[c], names + name_offsets[c + 1]); };
+    std::sort(order.begin(), order.end(), [&](uint32_t a, uint32_t b) {
+        if (first[a] != first[b]) return first[a] < first[b];
+        return name(a).compare(name(b)) < 0;
+    });
+    std::vector<uint32_t> tile_base(n_chroms, 0), contig_tiles(order.size());
+    uint64_t n_tiles = 0;
+    for (size_t i = 0; i < order.size(); ++i) {
+        contig_tiles[i] = (max_end[order[i]] - 1) / IGD_NBP + 1;
+        tile_base[order[i]] = (uint32_t)n_tiles;
+        n_tiles += contig_tiles[i];
+        if (n_tiles >= 0x7FFFFFFFull) return fail(GTGPU_ERR_UNSUPPORTED, "igd_serialize: 2^31 - 1 tiles or more");
+    }
+    const uint64_t n_ctg = order.size(), header_bytes = 12 + 4 * n_ctg + 4 * n_tiles + 40 * n_ctg;
+
+    std::unique_lock<std::mutex> glk;
+    if (!g->shards.empty()) glk = std::unique_lock<std::mutex>(ctx->group_mu);
+    std::lock_guard<std::mutex> lk(ctx->mu);
+    GT_CUDA(cudaSetDevice(ctx->device));
+    TempPool tp;
+    const uint64_t n = g->n_records;
+    int32_t *d_start = g->d_start, *d_end = g->d_end;
+    uint32_t *d_file = g->d_file, *d_chr;
+    if (g->shards.empty()) {
+        uint64_t* d_off64;
+        GT_TRY(tp.get(n, &d_chr));
+        GT_TRY(tp.get((uint64_t)n_chroms + 1, &d_off64));
+        const std::vector<uint64_t> off64(g->h_off.begin(), g->h_off.end());
+        GT_CUDA(cudaMemcpyAsync(d_off64, off64.data(), off64.size() * 8, cudaMemcpyHostToDevice, ctx->stream));
+        if (n) GT_TRY(launch_fill_set_ids(ctx, n_chroms, d_off64, d_chr));
+        GT_CUDA(cudaStreamSynchronize(ctx->stream));  // off64 is pageable
+    } else {
+        GT_TRY(igd_gather_shards(g, tp, &d_start, &d_end, &d_file, &d_chr));
+    }
+    BufPtr buf;
+    std::vector<uint32_t> tile_off;
+    GT_TRY(igd_write_tiles_locked(ctx, tp, n, d_start, d_end, d_file, d_chr, tile_base, n_tiles, header_bytes, &buf, &tile_off));
+
+    // the header: nbp, gType 1 (16-byte records), nCtg; nTile per contig; nCnt per tile; 40-byte NUL-padded names (igd.rs:418-486)
+    char* h = (char*)buf->block.ptr;
+    auto put = [&](int32_t v) {
+        memcpy(h, &v, 4);
+        h += 4;
+    };
+    put(IGD_NBP);
+    put(1);
+    put((int32_t)n_ctg);
+    for (uint32_t t : contig_tiles) put((int32_t)t);
+    for (uint64_t t = 0; t < n_tiles; ++t) put((int32_t)(tile_off[t + 1] - tile_off[t]));
+    for (uint32_t c : order) {
+        const uint32_t len = std::min<uint32_t>(name_offsets[c + 1] - name_offsets[c], 40);
+        memset(h, 0, 40);
+        memcpy(h, names + name_offsets[c], len);
+        h += 40;
+    }
+    *out_igd_bytes = buf.release();
+    return GTGPU_OK;
 } GT_CATCH

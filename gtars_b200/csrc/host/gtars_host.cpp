@@ -1015,6 +1015,25 @@ std::string with_extension(const std::string& path, const std::string& ext) {  /
     std::string stem = (dot == std::string::npos || (slash != std::string::npos && dot < slash) || dot == slash + 1) ? path : path.substr(0, dot);
     return stem + "." + ext;
 }
+// The companion .tsv (igd.rs:470-484): per file its index, name, region count and the average width to two decimals
+std::string igd_tsv(const std::vector<std::string>& names, const uint64_t* regions, const uint64_t* width_sums) {
+    std::string tsv = "Index\tFile\tNumber of Regions\tAvg size\n";
+    for (size_t f = 0; f < names.size(); ++f) {
+        char buf[64];
+        snprintf(buf, sizeof buf, "%.2f", regions[f] ? (double)width_sums[f] / (double)regions[f] : 0.0);
+        tsv += std::to_string(f) + "\t" + names[f] + "\t" + std::to_string(regions[f]) + "\t" + buf + "\n";
+    }
+    return tsv;
+}
+void write_igd_files(const std::string& path, const char* igd, size_t igd_bytes, const std::string& tsv) {
+    std::ofstream f(path, std::ios::binary);
+    if (!f) throw Error("cannot write " + path);
+    f.write(igd, (std::streamsize)igd_bytes);
+    if (!f) throw Error("cannot write " + path);
+    std::ofstream t(with_extension(path, "tsv"), std::ios::binary);
+    if (!t) throw Error("cannot write " + with_extension(path, "tsv"));
+    t << tsv;
+}
 }  // namespace
 
 void Igd::save_named_region_sets(const std::vector<std::pair<std::string, const RegionSet*>>& sets, const std::string& path, int32_t nbp) {
@@ -1022,15 +1041,15 @@ void Igd::save_named_region_sets(const std::vector<std::pair<std::string, const 
     std::vector<std::string> names;                       // contigs in creation order
     std::unordered_map<std::string, size_t> chrom_index;
     std::vector<std::vector<std::vector<IgdRec>>> contigs;  // [contig][tile][record]
-    std::string tsv = "Index\tFile\tNumber of Regions\tAvg size\n";
+    std::vector<std::string> file_names;
+    std::vector<uint64_t> regions(sets.size(), 0), width_sums(sets.size(), 0);
     for (size_t f = 0; f < sets.size(); ++f) {
-        uint32_t count = 0;
-        uint64_t total_width = 0;
+        file_names.push_back(sets[f].first);
         for (const Region& r : sets[f].second->regions) {
             if (!(r.start < r.end)) continue;
             const int32_t start = (int32_t)r.start, end = (int32_t)r.end;  // `as i32` casts (:295-296)
-            count += 1;
-            total_width += (uint64_t)(int64_t)(end - start);
+            regions[f] += 1;
+            width_sums[f] += (uint64_t)(int64_t)(int32_t)(r.end - r.start);
             if (start < 0 || end < 0 || start >= end) continue;  // Igd::add skips these silently
             auto it = chrom_index.find(r.chr);
             if (it == chrom_index.end()) {
@@ -1043,9 +1062,6 @@ void Igd::save_named_region_sets(const std::vector<std::pair<std::string, const 
             if (tiles.size() < (size_t)(n2 + 1)) tiles.resize((size_t)(n2 + 1));
             for (int32_t i = n1; i <= n2; ++i) tiles[i].push_back(IgdRec{(int32_t)f, start, end, 0});
         }
-        char buf[64];
-        snprintf(buf, sizeof buf, "%.2f", count ? (double)total_width / (double)count : 0.0);
-        tsv += std::to_string(f) + "\t" + sets[f].first + "\t" + std::to_string(count) + "\t" + buf + "\n";
     }
     std::string b;
     put_i32(b, nbp);
@@ -1065,12 +1081,20 @@ void Igd::save_named_region_sets(const std::vector<std::pair<std::string, const 
     for (auto& tiles : contigs)
         for (auto& t : tiles)
             for (const IgdRec& r : t) { put_i32(b, r.file_idx); put_i32(b, r.start); put_i32(b, r.end); put_i32(b, r.value); }
-    std::ofstream f(path, std::ios::binary);
-    if (!f) throw Error("cannot write " + path);
-    f.write(b.data(), (std::streamsize)b.size());
-    std::ofstream t(with_extension(path, "tsv"), std::ios::binary);
-    if (!t) throw Error("cannot write " + with_extension(path, "tsv"));
-    t << tsv;
+    write_igd_files(path, b.data(), b.size(), igd_tsv(file_names, regions.data(), width_sums.data()));
+}
+
+void Igd::save(const std::string& path, const std::vector<std::string>& names) const {
+    if (!igd_) throw Error("save needs a database Igd (not from_single_region_set)");
+    if (names.size() != n_files_)
+        throw Error("save: " + std::to_string(names.size()) + " names for " + std::to_string(n_files_) + " files");
+    NameBlob nb(cmap_);
+    PinnedResult bytes;
+    std::vector<uint64_t> regions(n_files_), width_sums(n_files_);
+    check(gtgpu_igd_serialize(igd_, (uint32_t)cmap_.size(), nb.blob.data(), nb.offsets.data(), &bytes.buf, regions.data(),
+                              width_sums.data()),
+          "gtgpu_igd_serialize");
+    write_igd_files(path, (const char*)gtgpu_buf_data(bytes.buf), gtgpu_buf_len(bytes.buf), igd_tsv(names, regions.data(), width_sums.data()));
 }
 
 std::unique_ptr<Igd> Igd::from_igd_file(std::shared_ptr<Device> dev, const std::string& path) {

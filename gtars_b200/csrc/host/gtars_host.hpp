@@ -264,6 +264,10 @@ class Igd {
     static void save_named_region_sets(const std::vector<std::pair<std::string, const RegionSet*>>& sets, const std::string& path,
                                        int32_t nbp = 16384);
     static std::unique_ptr<Igd> from_igd_file(std::shared_ptr<Device> dev, const std::string& path);
+    // Igd::save of this database (names[f] = file f's name in the .tsv): `path` (.igd) and the companion .tsv, the same bytes
+    // save_named_region_sets writes for the same sets, with the file built on the device (gtgpu_igd_serialize).  A database
+    // loaded with from_igd_file writes its kept records under the given names.  A database Igd only.
+    void save(const std::string& path, const std::vector<std::string>& names) const;
     // Igd(RegionSet::from_file(p) for p in paths) with every file's text parsed on the device (gtgpu_igd_build_bed): when every
     // path ends in ".gz" the gzip bytes go to the device inflater (gtgpu_igd_build_bed_gz), otherwise each file is read (".gz"
     // inflated by zlib) and the texts go back to back.  Chromosome ids follow the names' first appearance in the files.  Errors

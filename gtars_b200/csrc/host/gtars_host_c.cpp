@@ -300,6 +300,12 @@ int gth_igd_save_sets(uint64_t n, void** region_sets, const char** names, const 
         return 0;
     }, 1);
 }
+int gth_igd_save(void* g, uint64_t n, const char** names, const char* path) {
+    return guard([&]() -> int {
+        ((Igd*)g)->save(path, std::vector<std::string>(names, names + n));
+        return 0;
+    }, 1);
+}
 void* gth_igd_from_file(void* dev, const char* path) {
     return guard([&]() -> void* { return Igd::from_igd_file(*(std::shared_ptr<Device>*)dev, path).release(); }, nullptr);
 }

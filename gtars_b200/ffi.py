@@ -73,6 +73,7 @@ SIGNATURES = {
     "gtgpu_igd_build_bed": (_i32, [_vp, _u64, _vp, _vp, _vp, _vp, _vp, _vp]),
     "gtgpu_igd_build_bed_gz": (_i32, [_vp, _u64, _vp, _u64, _vp, _vp, _vp, _vp, _vp, _vp]),
     "gtgpu_igd_free": (_i32, [_vp]),
+    "gtgpu_igd_serialize": (_i32, [_vp, _u32, _vp, _vp, _vp, _vp, _vp]),
     "gtgpu_igd_info": (_i32, [_vp, _vp]),
     "gtgpu_igd_count_set_overlaps": (_i32, [_vp, _u64, _vp, _vp, _vp, _vp, _i32, _vp]),
     "gtgpu_igd_count_region_hits": (_i32, [_vp, _u64, _vp, _vp, _vp, _vp, _i32, _vp]),
@@ -618,6 +619,16 @@ class Igd:
 
     def count_region_hits(self, set_offsets, chr, start, end, min_overlap=1):
         return self._count(lib().gtgpu_igd_count_region_hits, set_offsets, chr, start, end, min_overlap)
+
+    def save_bytes(self, chrom_names):
+        """gtgpu_igd_serialize: (the .igd file's bytes as uint8, every file's region count, every file's width sum), the
+        database's chromosome i named chrom_names[i]."""
+        blob, offs = _names_blob(chrom_names)
+        regions = np.zeros(self.n_files, dtype=np.uint64)
+        widths = np.zeros(self.n_files, dtype=np.uint64)
+        h = C.c_void_p()
+        check(lib().gtgpu_igd_serialize(self._h, len(chrom_names), blob, _p(offs), C.byref(h), _p(regions), _p(widths)))
+        return _take(h, dtype=np.uint8), regions, widths
 
     def _count_bed(self, n_sets, chrom_names, call):
         blob, offs = _names_blob(chrom_names)

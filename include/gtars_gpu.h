@@ -365,6 +365,19 @@ int32_t gtgpu_igd_build_bed_gz(gtgpu_ctx* ctx, uint64_t n_files, const uint64_t*
                                const uint64_t* member_offsets, uint32_t* out_n_chroms, gtgpu_buf** out_chrom_names,
                                gtgpu_buf** out_chrom_name_offsets, gtgpu_igd** out_igd);
 int32_t gtgpu_igd_free(gtgpu_igd* igd);
+/* Igd::save (gtars-igd/src/igd.rs:418-486) of a database built any way (gtgpu_igd_build, gtgpu_igd_build_bed / _gz, one device
+ * or a group), written on the device: *out_igd_bytes (u8, gtgpu_buf_len = bytes) is the .igd file byte for byte as the
+ * reference writes it after Igd::from_named_region_sets over the same sets: nbp 16384, gType 1, the contigs in the order
+ * Igd::add created them (for gtgpu_igd_build: by the first kept record in the input arrays; for BED files, whose RegionSets the
+ * reference sorts by (name, start): by the first file with a kept record on the name, then by name bytes), a kept record in
+ * every tile it reaches, a tile stable-sorted by start, value 0.  Chromosomes without a kept record are not contigs.  The names
+ * are indexed by chromosome id, in the table format of gtgpu_igd_count_bed (n_names + 1 u32 byte offsets; a name is cut to 40
+ * bytes); n_names must equal the igd's chromosome count (else GTGPU_ERR_INVALID).  out_file_regions / out_file_width_sums
+ * (n_files each, caller-allocated) receive the .tsv numbers of every input file: its region lines with start < end as u32
+ * (records dropped as negative int32 included) and the wrapping u64 sum of their widths (int32 end - int32 start, widened);
+ * Avg size = sum / regions.  More than 2^32 - 2 tile entries give GTGPU_ERR_UNSUPPORTED. */
+int32_t gtgpu_igd_serialize(gtgpu_igd* igd, uint32_t n_names, const char* names, const uint32_t* name_offsets,
+                            gtgpu_buf** out_igd_bytes, uint64_t* out_file_regions, uint64_t* out_file_width_sums);
 /* info[0]=n_files, [1]=records kept, [2]=device bytes, [3]=lut shift */
 int32_t gtgpu_igd_info(const gtgpu_igd* igd, uint64_t info[4]);
 /* Igd::count_set_overlaps (igd.rs:544-556) / Igd::count_region_hits (igd.rs:563-590) for n_sets query sets at once:
