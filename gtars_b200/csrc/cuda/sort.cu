@@ -568,7 +568,8 @@ size_t radix_sort_temp_bytes(uint64_t n) {
     return (size_t)(table * 4 * 2 + exclusive_scan_temp_bytes(table, 4) + 256);
 }
 
-// Sorts by bits [0, bits) of the key.  keys/vals ping-pong between the a and b buffers; *result_in_b tells where the
+// Sorts by bits [0, bits) of the key; higher bits are ignored (except below bit 8: a single 8-bit pass for bits < 8 sorts by
+// bits [0, 8), callers pass keys < 2^bits).  keys/vals ping-pong between the a and b buffers; *result_in_b tells where the
 // sorted data ended up.  n < 2^32.
 // d_n (optional, device): the real element count when only the device knows it; n is then the capacity the grid is sized for.
 int32_t radix_sort_pairs(gtgpu_ctx* ctx, uint64_t n, uint32_t* keys_a, uint32_t* vals_a, uint32_t* keys_b, uint32_t* vals_b,
@@ -588,6 +589,9 @@ int32_t radix_sort_pairs(gtgpu_ctx* ctx, uint64_t n, uint32_t* keys_a, uint32_t*
     void* scan_tmp = starts + 512ull * cap_tiles;
     uint32_t *ki = keys_a, *vi = vals_a, *ko = keys_b, *vo = vals_b;
     for (int p = 0, shift = 0; p < passes; ++p, shift += width) {
+        // the last digit ends at bit `bits` (overlapping the one before it: the earlier passes already ordered the shared
+        // bits, so the stable pass keeps that order), so no key bit at or above `bits` takes part in the order
+        if (p == passes - 1 && passes > 1) shift = std::min(bits, 32) - width;
         int32_t status = GTGPU_OK;
         cudaError_t e = cudaErrorInvalidValue;
         switch (shape) {

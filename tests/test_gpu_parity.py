@@ -463,7 +463,8 @@ def test_fragments_random_differential(ctx, kind):
 def test_fragments_device_resident_entry_point(ctx, kind, style, n_bc):
     """gtgpu_tokenize_fragments_dev (no host copies, no synchronisation) and the host entry point against the oracle:
     lean universes, multi-hit universes (pool lists / generic walk under the per-query [unk] rule), barcode counts that
-    need one, two (9-bit digits) and three radix passes, degenerate and unknown-chromosome fragments, a partial last tile."""
+    take one 8-bit pair-sort pass (40) and the two-pass packed group-by with 8-bit (513) and 9-bit (70 000) low digits,
+    degenerate and unknown-chromosome fragments, a partial last tile.  Three and more passes: test_gpu_sort.py."""
     import torch
     rng = np.random.default_rng(zlib.crc32(f"fragdev/{kind}/{style}".encode()))
     n_chroms = 4
