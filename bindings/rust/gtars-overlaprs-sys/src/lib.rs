@@ -58,6 +58,15 @@ extern "C" {
                            out_start: *mut *mut gtgpu_buf, out_end: *mut *mut gtgpu_buf) -> i32;
     pub fn gtgpu_tokenize_bed(index: *mut gtgpu_index, text: *const u8, n_bytes: u64, n_names: u32, names: *const u8,
                               name_offsets: *const u32, unk_id: u32, out_ids: *mut *mut gtgpu_buf) -> i32;
+    /// Tokenizer::encode(RegionSet::try_from(file f)) for every file of a batch (file f = text[file_offsets[f], file_offsets[f + 1]),
+    /// any total size) in one device pass; out_file_token_offsets (n_files + 1) index *out_ids as in gtgpu_tokenize_files.
+    pub fn gtgpu_tokenize_bed_files(index: *mut gtgpu_index, n_files: u64, text: *const c_char, file_offsets: *const u64, n_names: u32,
+                                    names: *const u8, name_offsets: *const u32, unk_id: u32, out_file_token_offsets: *mut u64,
+                                    out_ids: *mut *mut gtgpu_buf) -> i32;
+    /// The same from gzip members: file f = members [file_members[f], file_members[f + 1]) of gz / member_offsets.
+    pub fn gtgpu_tokenize_bed_files_gz(index: *mut gtgpu_index, n_files: u64, file_members: *const u64, n_members: u64, gz: *const u8,
+                                       member_offsets: *const u64, n_names: u32, names: *const u8, name_offsets: *const u32,
+                                       unk_id: u32, out_file_token_offsets: *mut u64, out_ids: *mut *mut gtgpu_buf) -> i32;
     pub fn gtgpu_tokenize_fragments_text(index: *mut gtgpu_index, text: *const u8, n_bytes: u64, n_names: u32, names: *const u8,
                                          name_offsets: *const u32, unk_id: u32, out_n_barcodes: *mut u32,
                                          out_barcode_spans: *mut *mut gtgpu_buf, out_barcode_offsets: *mut *mut gtgpu_buf,

@@ -56,6 +56,7 @@ def lib():
             "gth_tokenizer_id_to_token": (cp, [vp, u32]), "gth_tokenizer_special": (cp, [vp, C.c_int]),
             "gth_tokenizer_kind": (C.c_int, [vp]), "gth_tokenizer_encode_batch": (vp, [vp, u64, vp]),
             "gth_tokenizer_fragments": (vp, [vp, cp]), "gth_tokenizer_fragments_device": (vp, [vp, cp]), "gth_tokenizer_encode_bed_file": (vp, [vp, cp]),
+            "gth_tokenizer_encode_bed_files": (vp, [vp, u64, vp]),
             "gth_parse_bed_file": (vp, [vp, cp, u64, vp]), "gth_gtok_write": (C.c_int, [cp, u64, vp, C.c_int]),
             "gth_gtok_read": (vp, [cp]),
             "gth_igd_single": (vp, [vp, vp]), "gth_igd_find_pairs": (vp, [vp, vp, i32]),
@@ -417,6 +418,12 @@ class Tokenizer:
     def encode_bed_file(self, path):
         """encode(RegionSet(path)) with the BED text parsed, sorted and tokenized on the device."""
         return _take_lists(lib().gth_tokenizer_encode_bed_file(self._h, os.fsencode(path)))[0]
+
+    def encode_bed_files(self, paths):
+        """[encode_bed_file(p) for p in paths] in one device pass over all the files' text, of any total size
+        (gtgpu_tokenize_bed_files; when every path ends in .gz the gzip bytes are inflated on the device too)."""
+        paths = [os.fsencode(p) for p in paths]
+        return _take_lists(lib().gth_tokenizer_encode_bed_files(self._h, len(paths), (C.c_char_p * max(len(paths), 1))(*paths)))
 
     def encode_batch(self, batches):
         """One Tokenizer::encode per element, all resolved in a single device pass."""

@@ -475,6 +475,16 @@ struct BedFilesRecords {
 };
 int32_t parse_bed_files_locked(gtgpu_ctx* ctx, const char* host_text, const char* dev_text, uint64_t n_files, const uint64_t* file_offsets,
                                const std::string& who, BedFilesRecords* out);
+// parse_bed_files_locked for query files: every record's chr in the ids of the caller's names (GTGPU_UNKNOWN_CHROM for a name
+// not among them).  *nt: the caller's name table in scratch SC_SET_ID (with_rank adds the names' ranks), uploaded when r->n > 0.
+int32_t parse_bed_queries_locked(gtgpu_ctx* ctx, const char* host_text, const char* dev_text, uint64_t n_files,
+                                 const uint64_t* file_offsets, uint32_t n_names, const char* names, const uint32_t* name_offsets,
+                                 bool with_rank, const std::string& who, BedFilesRecords* r, NameTable* nt);
+// gtgpu_tokenize_bed_files on text already split into n_files > 0 files (exactly one of host_text / dev_text is given):
+// out_file_token_offsets (n_files + 1, host) and *out_ids as gtgpu_tokenize_files returns them.
+int32_t tokenize_bed_files_locked(gtgpu_index* ix, const char* host_text, const char* dev_text, uint64_t n_files,
+                                  const uint64_t* file_offsets, uint32_t n_names, const char* names, const uint32_t* name_offsets,
+                                  uint32_t unk_id, const std::string& who, uint64_t* out_file_token_offsets, BufPtr* out_ids);
 
 // groups (api.cu, comm.cu, igd.cu)
 int32_t for_each_device(size_t n_devices, const std::function<int32_t(size_t)>& fn);

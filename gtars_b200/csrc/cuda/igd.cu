@@ -838,54 +838,7 @@ extern "C" int32_t gtgpu_igd_count_dev(gtgpu_igd* igd, int32_t binary, uint64_t 
     return igd_count_dev_locked(igd, binary != 0, n, d_set_of, d_chr, d_start, d_end, min_overlap, d_out);
 } GT_CATCH
 
-// ---- query sets from their BED files' text, parsed on the device ------------------------------------------------------------
-// parse_bed_files_locked numbers the query files' chromosome names in their first appearance; one launch maps every such name
-// to the database's id (the caller's name table, looked up as gtgpu_parse_bed does), one more rewrites every record's chr.
-namespace gtgpu {
-
-__global__ void igd_map_names_kernel(uint32_t n_names, const char* __restrict__ blob, const unsigned long long* __restrict__ offs,
-                                     NameTable nt, uint32_t* __restrict__ map) {
-    const uint32_t stride = gridDim.x * blockDim.x;
-    for (uint32_t i = blockIdx.x * blockDim.x + threadIdx.x; i < n_names; i += stride) {
-        const char* s = blob + offs[i];
-        const uint32_t len = (uint32_t)(offs[i + 1] - offs[i]);
-        map[i] = nt.lookup(fnv1a64(s, len), s, len);
-    }
-}
-
-__global__ void igd_remap_chr_kernel(uint64_t n, const uint32_t* __restrict__ map, uint32_t* __restrict__ chr) {
-    const uint64_t stride = (uint64_t)gridDim.x * blockDim.x;
-    for (uint64_t i = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += stride) chr[i] = map[chr[i]];
-}
-
-}  // namespace gtgpu
-
-// The query sets' records (set s = file s of the text, host_text or dev_text, file_offsets in bytes), their chr already in the
-// ids of the caller's names (GTGPU_UNKNOWN_CHROM for a name the database lacks).  The caller holds ctx->mu.
-static int32_t igd_parse_queries_locked(gtgpu_ctx* ctx, const char* host_text, const char* dev_text, uint64_t n_sets,
-                                        const uint64_t* file_offsets, uint32_t n_names, const char* names, const uint32_t* name_offsets,
-                                        const char* who, BedFilesRecords* r) {
-    GT_TRY(parse_bed_files_locked(ctx, host_text, dev_text, n_sets, file_offsets, who, r));
-    if (r->n == 0) return GTGPU_OK;
-    cudaStream_t st = ctx->stream;
-    NameTable nt;
-    GT_TRY(upload_name_table(ctx, n_names, names, name_offsets, &nt));  // scratch SC_SET_ID
-    const uint64_t blob_bytes = r->names->len;
-    DevMem d_blob, d_offs, d_map;
-    GT_TRY(d_blob.reserve(std::max<uint64_t>(blob_bytes, 1), 0, st));
-    GT_TRY(d_offs.reserve(((uint64_t)r->n_names + 1) * 8, 0, st));
-    GT_TRY(d_map.reserve((uint64_t)r->n_names * 4, 0, st));
-    if (blob_bytes) GT_CUDA(cudaMemcpyAsync(d_blob.ptr, r->names->block.ptr, blob_bytes, cudaMemcpyHostToDevice, st));
-    GT_CUDA(cudaMemcpyAsync(d_offs.ptr, r->name_offsets->block.ptr, ((uint64_t)r->n_names + 1) * 8, cudaMemcpyHostToDevice, st));
-    igd_map_names_kernel<<<grid_for(ctx, r->n_names), 256, 0, st>>>(r->n_names, (const char*)d_blob.ptr,
-                                                                      (const unsigned long long*)d_offs.ptr, nt, d_map.u32());
-    igd_remap_chr_kernel<<<grid_for(ctx, r->n), 256, 0, st>>>(r->n, d_map.u32(), r->chr.u32());
-    ctx->launches += 2;
-    GT_CUDA(cudaGetLastError());
-    GT_CUDA(cudaStreamSynchronize(st));  // the map is freed here, and a count may reuse the name table's scratch
-    return GTGPU_OK;
-}
-
+// ---- query sets from their BED files' text, parsed on the device (parse_bed_queries_locked) ---------------------------------
 // The parsed query sets against g.  One device counts the columns where the parse left them; a group runs its sharded count
 // with them as query arrays (each device pulls them from the first one) and gathers the shards' columns.
 static int32_t igd_count_parsed(gtgpu_igd* g, bool binary, uint64_t n_sets, const BedFilesRecords& r, int32_t m, uint64_t* out,
@@ -929,7 +882,9 @@ extern "C" int32_t gtgpu_igd_count_bed(gtgpu_igd* igd, int32_t binary, uint64_t 
     {
         std::lock_guard<std::mutex> lk(ctx->mu);
         GT_CUDA(cudaSetDevice(ctx->device));
-        GT_TRY(igd_parse_queries_locked(ctx, text, nullptr, n_sets, file_offsets, n_names, names, name_offsets, "igd_count_bed", &r));
+        NameTable nt;
+        GT_TRY(parse_bed_queries_locked(ctx, text, nullptr, n_sets, file_offsets, n_names, names, name_offsets, false, "igd_count_bed",
+                                        &r, &nt));
     }
     return igd_count_parsed(igd, binary != 0, n_sets, r, min_overlap, out, out_set_regions);
 } GT_CATCH
@@ -956,8 +911,9 @@ extern "C" int32_t gtgpu_igd_count_bed_gz(gtgpu_igd* igd, int32_t binary, uint64
         std::vector<uint64_t> text_offsets(n_members + 1), fo(n_sets + 1);
         GT_TRY(inflate_whole_locked(ctx, n_members, gz, member_offsets, "igd_count_bed_gz", &d_text, &n_text, text_offsets.data()));
         for (uint64_t s = 0; s <= n_sets; ++s) fo[s] = text_offsets[file_members[s]];
-        GT_TRY(igd_parse_queries_locked(ctx, nullptr, (const char*)d_text, n_sets, fo.data(), n_names, names, name_offsets,
-                                        "igd_count_bed_gz", &r));
+        NameTable nt;
+        GT_TRY(parse_bed_queries_locked(ctx, nullptr, (const char*)d_text, n_sets, fo.data(), n_names, names, name_offsets, false,
+                                        "igd_count_bed_gz", &r, &nt));
     }
     return igd_count_parsed(igd, binary != 0, n_sets, r, min_overlap, out, out_set_regions);
 } GT_CATCH

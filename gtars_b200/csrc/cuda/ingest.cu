@@ -192,31 +192,41 @@ __device__ __forceinline__ uint32_t rank_of(const uint32_t* __restrict__ name_ra
     return c < n_names ? name_rank[c] : n_names;  // unknown names after every known one
 }
 
+// The record kernels of the sort loop with 64-bit indices: a batch of files may hold up to 2^32 - 2 records, and a 32-bit
+// grid-stride index would wrap there.
+// file (optional): the records' file indices, grouped; a pair that straddles two files is in order whatever its keys
 __global__ void ingest_check_sorted_kernel(uint32_t n, const uint32_t* __restrict__ chr, const uint32_t* __restrict__ start,
-                                           const uint32_t* __restrict__ name_rank, uint32_t n_names, uint32_t* __restrict__ unsorted) {
-    const uint32_t stride = gridDim.x * blockDim.x;
-    for (uint32_t i = blockIdx.x * blockDim.x + threadIdx.x; i + 1 < n; i += stride) {
+                                           const uint32_t* __restrict__ name_rank, uint32_t n_names, uint32_t* __restrict__ unsorted,
+                                           const uint32_t* __restrict__ file = nullptr) {
+    const uint64_t stride = (uint64_t)gridDim.x * blockDim.x;
+    for (uint64_t i = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x; i + 1 < n; i += stride) {
+        if (file && file[i] != file[i + 1]) continue;
         const uint32_t ra = rank_of(name_rank, n_names, chr[i]), rb = rank_of(name_rank, n_names, chr[i + 1]);
         if (ra > rb || (ra == rb && start[i] > start[i + 1])) *unsorted = 1;
     }
 }
 
 __global__ void ingest_iota_kernel(uint32_t n, uint32_t* __restrict__ out) {
-    const uint32_t stride = gridDim.x * blockDim.x;
-    for (uint32_t i = blockIdx.x * blockDim.x + threadIdx.x; i < n; i += stride) out[i] = i;
+    const uint64_t stride = (uint64_t)gridDim.x * blockDim.x;
+    for (uint64_t i = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += stride) out[i] = (uint32_t)i;
 }
 
+// file (optional): the record's file index goes above the rank's rank_bits, so one pass orders by (file, rank)
 __global__ void ingest_rank_keys_kernel(uint32_t n, const uint32_t* __restrict__ order, const uint32_t* __restrict__ chr,
-                                        const uint32_t* __restrict__ name_rank, uint32_t n_names, uint32_t* __restrict__ keys) {
-    const uint32_t stride = gridDim.x * blockDim.x;
-    for (uint32_t i = blockIdx.x * blockDim.x + threadIdx.x; i < n; i += stride) keys[i] = rank_of(name_rank, n_names, chr[order[i]]);
+                                        const uint32_t* __restrict__ name_rank, uint32_t n_names, uint32_t* __restrict__ keys,
+                                        const uint32_t* __restrict__ file = nullptr, int rank_bits = 0) {
+    const uint64_t stride = (uint64_t)gridDim.x * blockDim.x;
+    for (uint64_t i = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += stride) {
+        const uint32_t j = order[i];
+        keys[i] = rank_of(name_rank, n_names, chr[j]) | (file ? file[j] << rank_bits : 0u);
+    }
 }
 
 __global__ void ingest_gather_kernel(uint32_t n, const uint32_t* __restrict__ order, const uint32_t* __restrict__ chr,
                                      const uint32_t* __restrict__ start, const uint32_t* __restrict__ end, uint32_t* __restrict__ o_chr,
                                      uint32_t* __restrict__ o_start, uint32_t* __restrict__ o_end) {
-    const uint32_t stride = gridDim.x * blockDim.x;
-    for (uint32_t i = blockIdx.x * blockDim.x + threadIdx.x; i < n; i += stride) {
+    const uint64_t stride = (uint64_t)gridDim.x * blockDim.x;
+    for (uint64_t i = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += stride) {
         const uint32_t j = order[i];
         o_chr[i] = chr[j];
         o_start[i] = start[j];
@@ -1098,6 +1108,127 @@ int32_t parse_bed_files_locked(gtgpu_ctx* ctx, const char* host_text, const char
     return GTGPU_OK;
 }
 
+// ---- query BED files: the discovered names mapped to the caller's ids ---------------------------------------------------------
+// parse_bed_files_locked numbers the files' chromosome names in their first appearance; one launch maps every such name to the
+// caller's id (its name table, looked up as gtgpu_parse_bed does), one more rewrites every record's chr.
+__global__ void ingest_map_names_kernel(uint32_t n_names, const char* __restrict__ blob, const unsigned long long* __restrict__ offs,
+                                        NameTable nt, uint32_t* __restrict__ map) {
+    const uint32_t stride = gridDim.x * blockDim.x;
+    for (uint32_t i = blockIdx.x * blockDim.x + threadIdx.x; i < n_names; i += stride) {
+        const char* s = blob + offs[i];
+        const uint32_t len = (uint32_t)(offs[i + 1] - offs[i]);
+        map[i] = nt.lookup(fnv1a64(s, len), s, len);
+    }
+}
+
+__global__ void ingest_remap_chr_kernel(uint64_t n, const uint32_t* __restrict__ map, uint32_t* __restrict__ chr) {
+    const uint64_t stride = (uint64_t)gridDim.x * blockDim.x;
+    for (uint64_t i = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += stride) chr[i] = map[chr[i]];
+}
+
+int32_t parse_bed_queries_locked(gtgpu_ctx* ctx, const char* host_text, const char* dev_text, uint64_t n_files,
+                                 const uint64_t* file_offsets, uint32_t n_names, const char* names, const uint32_t* name_offsets,
+                                 bool with_rank, const std::string& who, BedFilesRecords* r, NameTable* nt) {
+    GT_TRY(parse_bed_files_locked(ctx, host_text, dev_text, n_files, file_offsets, who, r));
+    if (r->n == 0) return GTGPU_OK;
+    cudaStream_t st = ctx->stream;
+    GT_TRY(upload_name_table(ctx, n_names, names, name_offsets, nt, with_rank));  // scratch SC_SET_ID
+    const uint64_t blob_bytes = r->names->len;
+    DevMem d_blob, d_offs, d_map;
+    GT_TRY(d_blob.reserve(std::max<uint64_t>(blob_bytes, 1), 0, st));
+    GT_TRY(d_offs.reserve(((uint64_t)r->n_names + 1) * 8, 0, st));
+    GT_TRY(d_map.reserve((uint64_t)r->n_names * 4, 0, st));
+    if (blob_bytes) GT_CUDA(cudaMemcpyAsync(d_blob.ptr, r->names->block.ptr, blob_bytes, cudaMemcpyHostToDevice, st));
+    GT_CUDA(cudaMemcpyAsync(d_offs.ptr, r->name_offsets->block.ptr, ((uint64_t)r->n_names + 1) * 8, cudaMemcpyHostToDevice, st));
+    ingest_map_names_kernel<<<igrid(ctx, r->n_names), 256, 0, st>>>(r->n_names, (const char*)d_blob.ptr,
+                                                                     (const unsigned long long*)d_offs.ptr, *nt, d_map.u32());
+    ingest_remap_chr_kernel<<<igrid(ctx, r->n), 256, 0, st>>>(r->n, d_map.u32(), r->chr.u32());
+    ctx->launches += 2;
+    GT_CUDA(cudaGetLastError());
+    GT_CUDA(cudaStreamSynchronize(st));  // the map is freed here, and a later call may reuse the name table's scratch
+    return GTGPU_OK;
+}
+
+// ---- a batch of BED files tokenized in one pass: parse, per-file RegionSet::sort, fused find, [unk] rule ----------------------
+// The records arrive grouped by file in file order.  RegionSet::sort applies per file: stable by (chromosome string, start).  When
+// some file is out of order, stable radix passes by start, then chromosome rank, then file index (folded into the rank pass when
+// both fit 32 bits) give every file its own records in that order.  The caller holds ctx->mu.
+int32_t tokenize_bed_files_locked(gtgpu_index* ix, const char* host_text, const char* dev_text, uint64_t n_files,
+                                  const uint64_t* file_offsets, uint32_t n_names, const char* names, const uint32_t* name_offsets,
+                                  uint32_t unk_id, const std::string& who, uint64_t* out_file_token_offsets, BufPtr* out_ids) {
+    gtgpu_ctx* ctx = ix->ctx;
+    cudaStream_t st = ctx->stream;
+    BedFilesRecords r;
+    NameTable nt{};
+    GT_TRY(parse_bed_queries_locked(ctx, host_text, dev_text, n_files, file_offsets, n_names, names, name_offsets, true, who, &r, &nt));
+    const uint32_t n = (uint32_t)r.n;  // parse_bed_files_locked allows fewer than 2^32 - 1 records
+    const uint32_t *q_chr = r.chr.u32(), *q_start = r.start.u32(), *q_end = r.end.u32();
+    uint32_t* d_flag;
+    GT_TRY(ctx->scratch_get(SC_MISC, 64, (void**)&d_flag));
+    GT_CUDA(cudaMemsetAsync(d_flag, 0, 4, st));
+    ingest_check_sorted_kernel<<<igrid(ctx, n), 256, 0, st>>>(n, q_chr, q_start, nt.rank, n_names, d_flag, r.file.u32());
+    ctx->launches++;
+    uint32_t unsorted = 0;
+    GT_CUDA(cudaMemcpyAsync(&unsorted, d_flag, 4, cudaMemcpyDeviceToHost, st));
+    GT_CUDA(cudaStreamSynchronize(st));
+    if (unsorted) {  // the parse's line scratch is free again; the find below does not touch it
+        uint32_t *k_a, *v_a, *k_b, *v_b;
+        GT_TRY(ctx->scratch_get(SC_ING_0, (size_t)n * 4, (void**)&k_a));
+        GT_TRY(ctx->scratch_get(SC_ING_1, (size_t)n * 4, (void**)&v_a));
+        GT_TRY(ctx->scratch_get(SC_ING_2, (size_t)n * 4, (void**)&k_b));
+        GT_TRY(ctx->scratch_get(SC_ING_3, (size_t)n * 4, (void**)&v_b));
+        void* d_tmp;
+        GT_TRY(ctx->scratch_get(SC_IN3_START, radix_sort_temp_bytes(n), &d_tmp));
+        GT_CUDA(cudaMemcpyAsync(k_a, q_start, (size_t)n * 4, cudaMemcpyDeviceToDevice, st));
+        ingest_iota_kernel<<<igrid(ctx, n), 256, 0, st>>>(n, v_a);
+        ctx->launches++;
+        int in_b = 0;
+        GT_TRY(radix_sort_pairs(ctx, n, k_a, v_a, k_b, v_b, 32, d_tmp, &in_b));
+        if (in_b) { std::swap(k_a, k_b); std::swap(v_a, v_b); }
+        int rank_bits = 1, file_bits = 1;
+        while (rank_bits < 32 && (1ull << rank_bits) < (uint64_t)n_names + 1) ++rank_bits;
+        while (file_bits < 32 && (1ull << file_bits) < n_files) ++file_bits;
+        const bool fold = rank_bits + file_bits <= 32;
+        ingest_rank_keys_kernel<<<igrid(ctx, n), 256, 0, st>>>(n, v_a, q_chr, nt.rank, n_names, k_a, fold ? r.file.u32() : nullptr,
+                                                              rank_bits);
+        ctx->launches++;
+        GT_TRY(radix_sort_pairs(ctx, n, k_a, v_a, k_b, v_b, fold ? rank_bits + file_bits : rank_bits, d_tmp, &in_b));
+        if (in_b) { std::swap(k_a, k_b); std::swap(v_a, v_b); }
+        if (!fold) {
+            GT_TRY(launch_gather_u32(ctx, n, r.file.u32(), v_a, k_a));
+            GT_TRY(radix_sort_pairs(ctx, n, k_a, v_a, k_b, v_b, file_bits, d_tmp, &in_b));
+            if (in_b) { std::swap(k_a, k_b); std::swap(v_a, v_b); }
+        }
+        // the order is v_a; the other three buffers take the sorted columns
+        ingest_gather_kernel<<<igrid(ctx, n), 256, 0, st>>>(n, v_a, q_chr, q_start, q_end, k_a, k_b, v_b);
+        ctx->launches++;
+        q_chr = k_a; q_start = k_b; q_end = v_b;
+    }
+    // ---- fused find over the files, then the [unk] rule (Tokenizer::tokenize: a file without a token yields [unk]) ----------------
+    uint64_t *d_fo, *d_raw_tok, *d_out_tok, total = 0;
+    GT_TRY(ctx->scratch_get(SC_FILE_OFFS, (n_files + 1) * 8, (void**)&d_fo));
+    GT_TRY(ctx->scratch_get(SC_FILE_TOK, (n_files + 1) * 8, (void**)&d_raw_tok));
+    GT_TRY(ctx->scratch_get(SC_FILE_TOK2, (n_files + 1) * 8, (void**)&d_out_tok));
+    GT_CUDA(cudaMemcpyAsync(d_fo, r.file_offsets.data(), (n_files + 1) * 8, cudaMemcpyHostToDevice, st));
+    uint32_t *d_ids = nullptr, *d_ids2 = nullptr;
+    GT_TRY(fused_find_all(ix, n, n_files, d_fo, q_chr, q_start, q_end, nullptr, d_raw_tok, &d_ids, &total));  // synchronises
+    uint64_t* d_misc;
+    GT_TRY(ctx->scratch_get(SC_MISC, 64, (void**)&d_misc));
+    GT_TRY(ctx->scratch_get(SC_OUT_IDS2, (total + n_files) * 4 + 4, (void**)&d_ids2));
+    GT_TRY(launch_unk_offsets(ctx, n_files, d_raw_tok, d_out_tok, d_misc + 1));
+    GT_TRY(launch_unk_expand(ctx, n_files, d_raw_tok, d_out_tok, d_ids, unk_id, d_ids2));
+    GT_CUDA(cudaMemcpyAsync(out_file_token_offsets, d_out_tok, (n_files + 1) * 8, cudaMemcpyDeviceToHost, st));
+    GT_CUDA(cudaStreamSynchronize(st));
+    BufPtr buf;
+    int32_t s = buf_from_device(ctx, d_ids2, out_file_token_offsets[n_files], 4, st, &buf);
+    if (s == GTGPU_ERR_CUDA) return fail(s, who + ": D2H: " + gtgpu_last_error());
+    GT_TRY(s);
+    const cudaError_t e = cudaStreamSynchronize(st);
+    if (e != cudaSuccess) return fail(GTGPU_ERR_CUDA, who + ": D2H: " + cudaGetErrorString(e));
+    *out_ids = std::move(buf);
+    return GTGPU_OK;
+}
+
 }  // namespace gtgpu
 
 using namespace gtgpu;
@@ -1161,6 +1292,64 @@ int32_t gtgpu::tokenize_bed_locked(gtgpu_index* ix, const char* host_text, const
     *out_ids = buf.release();
     return GTGPU_OK;
 }
+
+// n_files == 0: the offsets are [0] and the id buffer is empty
+static int32_t tokenize_no_files(gtgpu_ctx* ctx, uint64_t* out_file_token_offsets, gtgpu_buf** out_ids) {
+    BufPtr buf;
+    GT_TRY(buf_new(ctx, 0, 4, &buf));
+    out_file_token_offsets[0] = 0;
+    *out_ids = buf.release();
+    return GTGPU_OK;
+}
+
+extern "C" int32_t gtgpu_tokenize_bed_files(gtgpu_index* ix, uint64_t n_files, const char* text, const uint64_t* file_offsets,
+                                            uint32_t n_names, const char* names, const uint32_t* name_offsets, uint32_t unk_id,
+                                            uint64_t* out_file_token_offsets, gtgpu_buf** out_ids) try {
+    if (!ix || !file_offsets || !out_file_token_offsets || !out_ids || (n_names && (!names || !name_offsets)))
+        return fail(GTGPU_ERR_INVALID, "tokenize_bed_files: null argument");
+    if (file_offsets[0] != 0) return fail(GTGPU_ERR_INVALID, "tokenize_bed_files: file_offsets[0] must be 0");
+    for (uint64_t f = 0; f < n_files; ++f)
+        if (file_offsets[f] > file_offsets[f + 1]) return fail(GTGPU_ERR_INVALID, "tokenize_bed_files: file_offsets not monotone");
+    if (file_offsets[n_files] && !text) return fail(GTGPU_ERR_INVALID, "tokenize_bed_files: null text");
+    if (n_files >= 0xFFFFFFFFull) return fail(GTGPU_ERR_UNSUPPORTED, "tokenize_bed_files: too many files");
+    gtgpu_ctx* ctx = ix->ctx;
+    std::lock_guard<std::mutex> lk(ctx->mu);
+    GT_CUDA(cudaSetDevice(ctx->device));
+    if (n_files == 0) return tokenize_no_files(ctx, out_file_token_offsets, out_ids);
+    BufPtr ids;
+    GT_TRY(tokenize_bed_files_locked(ix, text, nullptr, n_files, file_offsets, n_names, names, name_offsets, unk_id, "tokenize_bed_files",
+                                     out_file_token_offsets, &ids));
+    *out_ids = ids.release();
+    return GTGPU_OK;
+} GT_CATCH
+
+extern "C" int32_t gtgpu_tokenize_bed_files_gz(gtgpu_index* ix, uint64_t n_files, const uint64_t* file_members, uint64_t n_members,
+                                               const uint8_t* gz, const uint64_t* member_offsets, uint32_t n_names, const char* names,
+                                               const uint32_t* name_offsets, uint32_t unk_id, uint64_t* out_file_token_offsets,
+                                               gtgpu_buf** out_ids) try {
+    if (!ix || !file_members || !out_file_token_offsets || !out_ids || (n_names && (!names || !name_offsets)))
+        return fail(GTGPU_ERR_INVALID, "tokenize_bed_files_gz: null argument");
+    GT_TRY(check_members(n_members, gz, member_offsets, "tokenize_bed_files_gz"));
+    if (file_members[0] != 0 || file_members[n_files] != n_members)
+        return fail(GTGPU_ERR_INVALID, "tokenize_bed_files_gz: file_members must run from 0 to n_members");
+    for (uint64_t f = 0; f < n_files; ++f)
+        if (file_members[f] > file_members[f + 1]) return fail(GTGPU_ERR_INVALID, "tokenize_bed_files_gz: file_members not monotone");
+    if (n_files >= 0xFFFFFFFFull) return fail(GTGPU_ERR_UNSUPPORTED, "tokenize_bed_files_gz: too many files");
+    gtgpu_ctx* ctx = ix->ctx;
+    std::lock_guard<std::mutex> lk(ctx->mu);
+    GT_CUDA(cudaSetDevice(ctx->device));
+    if (n_files == 0) return tokenize_no_files(ctx, out_file_token_offsets, out_ids);
+    uint8_t* d_text = nullptr;
+    uint64_t n_text = 0;
+    std::vector<uint64_t> text_offsets(n_members + 1), fo(n_files + 1);
+    GT_TRY(inflate_whole_locked(ctx, n_members, gz, member_offsets, "tokenize_bed_files_gz", &d_text, &n_text, text_offsets.data()));
+    for (uint64_t f = 0; f <= n_files; ++f) fo[f] = text_offsets[file_members[f]];
+    BufPtr ids;
+    GT_TRY(tokenize_bed_files_locked(ix, nullptr, (const char*)d_text, n_files, fo.data(), n_names, names, name_offsets, unk_id,
+                                     "tokenize_bed_files_gz", out_file_token_offsets, &ids));
+    *out_ids = ids.release();
+    return GTGPU_OK;
+} GT_CATCH
 
 // tokenize_fragment_file (fragments.rs:61-82) from the file's text, < 4 GiB: the barcodes come back as u32 spans into the text.
 extern "C" int32_t gtgpu_tokenize_fragments_text(gtgpu_index* ix, const char* text, uint64_t n_bytes, uint32_t n_names,

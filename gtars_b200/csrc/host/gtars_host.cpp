@@ -642,6 +642,80 @@ static bool gz_members_for_device(const std::string& path, std::string& raw, std
     return true;
 }
 
+namespace {
+// The bytes of n BED files for one device call.  When every path ends in ".gz" they stay gzip: every file's bytes back to back
+// with their member offsets, for the device inflater.  Otherwise the texts go back to back (".gz" inflated by zlib).
+struct BedFilesBytes {
+    bool gz = false;
+    std::string raw;                                   // gz: the files' gzip bytes
+    std::vector<uint64_t> members{0}, file_members{0};  // gz: member offsets in raw; file f = members [file_members[f], [f + 1])
+    std::unique_ptr<char[]> text;                      // otherwise: the texts, file f = text[file_offsets[f], file_offsets[f + 1])
+    std::vector<uint64_t> file_offsets{0};
+};
+
+BedFilesBytes gather_bed_files(const std::vector<std::string>& paths) {
+    BedFilesBytes b;
+    if (!paths.empty() && std::all_of(paths.begin(), paths.end(), ends_with_gz)) {
+        // one-member .bed.gz files are the common case: every member of every file is inflated on the device in parallel
+        b.gz = true;
+        std::string raw;
+        std::vector<uint64_t> m;
+        for (const auto& p : paths) {
+            read_raw_bytes(p, raw);
+            uint64_t n = 0;
+            gtgpu_gzip_members((const uint8_t*)raw.data(), raw.size(), 0, nullptr, &n);  // count only
+            m.assign(n + 1, 0);
+            check(gtgpu_gzip_members((const uint8_t*)raw.data(), raw.size(), m.size(), m.data(), &n), "gtgpu_gzip_members");
+            for (uint64_t k = 1; k <= n; ++k) b.members.push_back(b.raw.size() + m[k]);
+            b.file_members.push_back(b.members.size() - 1);
+            b.raw += raw;
+        }
+        return b;
+    }
+    // the texts back to back; the library stages them to the device through its own pinned blocks
+    std::vector<std::string> inflated(paths.size());
+    for (size_t f = 0; f < paths.size(); ++f) {
+        uint64_t size = 0;
+        if (ends_with_gz(paths[f])) {
+            inflated[f] = read_file_bytes(paths[f]);
+            size = inflated[f].size();
+        } else {
+            std::ifstream in(paths[f], std::ios::binary | std::ios::ate);
+            if (!in) throw Error("Failed to open file: \"" + paths[f] + "\"");
+            size = (uint64_t)std::max<std::streamsize>(in.tellg(), 0);
+        }
+        b.file_offsets.push_back(b.file_offsets.back() + size);
+    }
+    b.text.reset(new char[std::max<uint64_t>(b.file_offsets.back(), 1)]);
+    for (size_t f = 0; f < paths.size(); ++f) {
+        char* dst = b.text.get() + b.file_offsets[f];
+        const uint64_t size = b.file_offsets[f + 1] - b.file_offsets[f];
+        if (ends_with_gz(paths[f])) {
+            memcpy(dst, inflated[f].data(), size);
+            std::string().swap(inflated[f]);
+        } else if (size) {
+            std::ifstream in(paths[f], std::ios::binary);
+            if (!in || !in.read(dst, (std::streamsize)size)) throw Error("Failed to read file: \"" + paths[f] + "\"");
+        }
+    }
+    return b;
+}
+
+// The library's last error as "fn: message", "file k" in it replaced by the file's path
+[[noreturn]] void throw_naming_path(const char* fn, const std::vector<std::string>& paths) {
+    std::string msg = gtgpu_last_error();
+    const size_t k = msg.find(": file ");
+    size_t b = k == std::string::npos ? k : k + 7;
+    if (b != std::string::npos) {
+        const size_t a = b;
+        while (b < msg.size() && isdigit((unsigned char)msg[b])) ++b;
+        if (b > a && std::stoull(msg.substr(a, b - a)) < paths.size())
+            msg = msg.substr(0, k) + ": \"" + paths[std::stoull(msg.substr(a, b - a))] + "\"" + msg.substr(b);
+    }
+    throw Error(std::string(fn) + ": " + msg);
+}
+}  // namespace
+
 std::vector<uint32_t> Tokenizer::encode_bed_file(const std::string& path) const {
     NameBlob nb(cmap_);
     PinnedResult ids;
@@ -658,6 +732,29 @@ std::vector<uint32_t> Tokenizer::encode_bed_file(const std::string& path) const 
                              &ids.buf),
           "gtgpu_tokenize_bed");
     return std::vector<uint32_t>(ids.data(), ids.data() + ids.len());
+}
+
+std::vector<std::vector<uint32_t>> Tokenizer::encode_bed_files(const std::vector<std::string>& paths) const {
+    const BedFilesBytes b = gather_bed_files(paths);
+    NameBlob nb(cmap_);
+    std::vector<uint64_t> tok_offsets(paths.size() + 1);
+    PinnedResult ids;
+    int32_t status;
+    const char* fn;
+    if (b.gz) {
+        fn = "gtgpu_tokenize_bed_files_gz";
+        status = gtgpu_tokenize_bed_files_gz(index_, paths.size(), b.file_members.data(), b.members.size() - 1, (const uint8_t*)b.raw.data(),
+                                             b.members.data(), (uint32_t)cmap_.size(), nb.blob.data(), nb.offsets.data(), unk_id_,
+                                             tok_offsets.data(), &ids.buf);
+    } else {
+        fn = "gtgpu_tokenize_bed_files";
+        status = gtgpu_tokenize_bed_files(index_, paths.size(), b.text.get(), b.file_offsets.data(), (uint32_t)cmap_.size(),
+                                          nb.blob.data(), nb.offsets.data(), unk_id_, tok_offsets.data(), &ids.buf);
+    }
+    if (status != GTGPU_OK) throw_naming_path(fn, paths);
+    std::vector<std::vector<uint32_t>> out(paths.size());
+    for (size_t f = 0; f < paths.size(); ++f) out[f].assign(ids.data() + tok_offsets[f], ids.data() + tok_offsets[f + 1]);
+    return out;
 }
 
 std::vector<std::string> Tokenizer::tokenize(const std::vector<Region>& regions) const {
@@ -1169,80 +1266,6 @@ std::unique_ptr<Igd> Igd::from_igd_file(std::shared_ptr<Device> dev, const std::
           "gtgpu_igd_build");
     return g;
 }
-
-namespace {
-// The bytes of n BED files for one device call.  When every path ends in ".gz" they stay gzip: every file's bytes back to back
-// with their member offsets, for the device inflater.  Otherwise the texts go back to back (".gz" inflated by zlib).
-struct BedFilesBytes {
-    bool gz = false;
-    std::string raw;                                   // gz: the files' gzip bytes
-    std::vector<uint64_t> members{0}, file_members{0};  // gz: member offsets in raw; file f = members [file_members[f], [f + 1])
-    std::unique_ptr<char[]> text;                      // otherwise: the texts, file f = text[file_offsets[f], file_offsets[f + 1])
-    std::vector<uint64_t> file_offsets{0};
-};
-
-BedFilesBytes gather_bed_files(const std::vector<std::string>& paths) {
-    BedFilesBytes b;
-    if (!paths.empty() && std::all_of(paths.begin(), paths.end(), ends_with_gz)) {
-        // one-member .bed.gz files are the common case: every member of every file is inflated on the device in parallel
-        b.gz = true;
-        std::string raw;
-        std::vector<uint64_t> m;
-        for (const auto& p : paths) {
-            read_raw_bytes(p, raw);
-            uint64_t n = 0;
-            gtgpu_gzip_members((const uint8_t*)raw.data(), raw.size(), 0, nullptr, &n);  // count only
-            m.assign(n + 1, 0);
-            check(gtgpu_gzip_members((const uint8_t*)raw.data(), raw.size(), m.size(), m.data(), &n), "gtgpu_gzip_members");
-            for (uint64_t k = 1; k <= n; ++k) b.members.push_back(b.raw.size() + m[k]);
-            b.file_members.push_back(b.members.size() - 1);
-            b.raw += raw;
-        }
-        return b;
-    }
-    // the texts back to back; the library stages them to the device through its own pinned blocks
-    std::vector<std::string> inflated(paths.size());
-    for (size_t f = 0; f < paths.size(); ++f) {
-        uint64_t size = 0;
-        if (ends_with_gz(paths[f])) {
-            inflated[f] = read_file_bytes(paths[f]);
-            size = inflated[f].size();
-        } else {
-            std::ifstream in(paths[f], std::ios::binary | std::ios::ate);
-            if (!in) throw Error("Failed to open file: \"" + paths[f] + "\"");
-            size = (uint64_t)std::max<std::streamsize>(in.tellg(), 0);
-        }
-        b.file_offsets.push_back(b.file_offsets.back() + size);
-    }
-    b.text.reset(new char[std::max<uint64_t>(b.file_offsets.back(), 1)]);
-    for (size_t f = 0; f < paths.size(); ++f) {
-        char* dst = b.text.get() + b.file_offsets[f];
-        const uint64_t size = b.file_offsets[f + 1] - b.file_offsets[f];
-        if (ends_with_gz(paths[f])) {
-            memcpy(dst, inflated[f].data(), size);
-            std::string().swap(inflated[f]);
-        } else if (size) {
-            std::ifstream in(paths[f], std::ios::binary);
-            if (!in || !in.read(dst, (std::streamsize)size)) throw Error("Failed to read file: \"" + paths[f] + "\"");
-        }
-    }
-    return b;
-}
-
-// The library's last error as "fn: message", "file k" in it replaced by the file's path
-[[noreturn]] void throw_naming_path(const char* fn, const std::vector<std::string>& paths) {
-    std::string msg = gtgpu_last_error();
-    const size_t k = msg.find(": file ");
-    size_t b = k == std::string::npos ? k : k + 7;
-    if (b != std::string::npos) {
-        const size_t a = b;
-        while (b < msg.size() && isdigit((unsigned char)msg[b])) ++b;
-        if (b > a && std::stoull(msg.substr(a, b - a)) < paths.size())
-            msg = msg.substr(0, k) + ": \"" + paths[std::stoull(msg.substr(a, b - a))] + "\"" + msg.substr(b);
-    }
-    throw Error(std::string(fn) + ": " + msg);
-}
-}  // namespace
 
 std::unique_ptr<Igd> Igd::from_bed_files(std::shared_ptr<Device> dev, const std::vector<std::string>& paths) {
     std::unique_ptr<Igd> g(new Igd());

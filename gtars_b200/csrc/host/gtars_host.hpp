@@ -208,6 +208,9 @@ class Tokenizer {
     std::vector<uint32_t> encode(const std::vector<Region>& regions) const;       // tokenizer.rs:165-171
     // encode(RegionSet::try_from(path)) with the file's text parsed, sorted and tokenized on the device (gtgpu_tokenize_bed).
     std::vector<uint32_t> encode_bed_file(const std::string& path) const;
+    // encode_bed_file(paths[f]) for every f in ONE device pass over all the files' text, of any total size
+    // (gtgpu_tokenize_bed_files; gtgpu_tokenize_bed_files_gz when every path ends in ".gz").
+    std::vector<std::vector<uint32_t>> encode_bed_files(const std::vector<std::string>& paths) const;
     // One encode() per region set, resolved in ONE device pass (the batch shape the GPU serves).
     std::vector<std::vector<uint32_t>> encode_batch(const std::vector<const std::vector<Region>*>& calls) const;
     std::vector<std::string> decode(const std::vector<uint32_t>& ids) const;      // tokenizer.rs:173-181

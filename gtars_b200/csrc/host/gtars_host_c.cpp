@@ -197,6 +197,14 @@ void* gth_tokenizer_encode_bed_file(void* t, const char* path) {
         return l;
     }, nullptr);
 }
+void* gth_tokenizer_encode_bed_files(void* t, uint64_t n, const char** paths) {
+    return guard([&]() -> void* {
+        auto lists = ((Tokenizer*)t)->encode_bed_files(std::vector<std::string>(paths, paths + n));
+        Lists* l = new Lists();
+        l->lists = std::move(lists);
+        return l;
+    }, nullptr);
+}
 // BED text -> (chr ids, starts, ends) through the device parser; chromosome names in `names` (n of them) get ids 0..n-1
 void* gth_parse_bed_file(void* dev, const char* path, uint64_t n_names, const char** names) {
     return guard([&]() -> void* {

@@ -55,6 +55,8 @@ SIGNATURES = {
     "gtgpu_tokenize_fragments_dev": (_i32, [_vp, _u64, _vp, _vp, _vp, _vp, _u32, _u32, _vp, _vp, _u64, _vp]),
     "gtgpu_parse_bed": (_i32, [_vp, _vp, _u64, _u32, _vp, _vp, _vp, _vp, _vp, _vp]),
     "gtgpu_tokenize_bed": (_i32, [_vp, _vp, _u64, _u32, _vp, _vp, _u32, _vp]),
+    "gtgpu_tokenize_bed_files": (_i32, [_vp, _u64, _vp, _vp, _u32, _vp, _vp, _u32, _vp, _vp]),
+    "gtgpu_tokenize_bed_files_gz": (_i32, [_vp, _u64, _vp, _u64, _vp, _vp, _u32, _vp, _vp, _u32, _vp, _vp]),
     "gtgpu_tokenize_fragments_text": (_i32, [_vp, _vp, _u64, _u32, _vp, _vp, _u32, _vp, _vp, _vp, _vp]),
     "gtgpu_gzip_members": (_i32, [_vp, _u64, _u64, _vp, _vp]),
     "gtgpu_gunzip": (_i32, [_vp, _u64, _vp, _vp, _vp, _vp]),
@@ -361,6 +363,28 @@ class Index:
         h = C.c_void_p()
         check(lib().gtgpu_tokenize_bed_gz(self._h, len(mo) - 1, gz, _p(mo), len(chrom_names), blob, _p(offs), unk_id, C.byref(h)))
         return _take(h)
+
+    def tokenize_bed_files(self, text, file_offsets, chrom_names, unk_id):
+        """gtgpu_tokenize_bed_files: file f = text[file_offsets[f]:file_offsets[f + 1]] parsed, sorted per file and tokenized on
+        the device.  Returns (file_token_offsets, ids) as tokenize_files does.  `text` may be a uint8 numpy array."""
+        fo = _arr(file_offsets, np.uint64)
+        blob, offs = _names_blob(chrom_names)
+        out_off = np.empty(len(fo), dtype=np.uint64)
+        h = C.c_void_p()
+        check(lib().gtgpu_tokenize_bed_files(self._h, len(fo) - 1, _text_ptr(text), _p(fo), len(chrom_names), blob, _p(offs), unk_id,
+                                             _p(out_off), C.byref(h)))
+        return out_off, _take(h)
+
+    def tokenize_bed_files_gz(self, gz, file_members, member_offsets, chrom_names, unk_id):
+        """gtgpu_tokenize_bed_files_gz: file f = gzip members [file_members[f], file_members[f + 1]) of `gz` (member_offsets as
+        gzip_members returns them), inflated, parsed, sorted per file and tokenized on the device."""
+        fm, mo = _arr(file_members, np.uint64), _arr(member_offsets, np.uint64)
+        blob, offs = _names_blob(chrom_names)
+        out_off = np.empty(len(fm), dtype=np.uint64)
+        h = C.c_void_p()
+        check(lib().gtgpu_tokenize_bed_files_gz(self._h, len(fm) - 1, _p(fm), len(mo) - 1, _text_ptr(gz), _p(mo), len(chrom_names),
+                                                blob, _p(offs), unk_id, _p(out_off), C.byref(h)))
+        return out_off, _take(h)
 
     def tokenize_fragments_text(self, text: bytes, chrom_names, unk_id, gz_member_offsets=None):
         """gtgpu_tokenize_fragments_text (or _gz when gz_member_offsets is given: `text` is then the gzip data):

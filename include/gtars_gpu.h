@@ -224,6 +224,24 @@ int32_t gtgpu_parse_bed(gtgpu_ctx* ctx, const char* text, uint64_t n_bytes, uint
                         gtgpu_buf** out_end);
 int32_t gtgpu_tokenize_bed(gtgpu_index* index, const char* text, uint64_t n_bytes, uint32_t n_names, const char* names,
                            const uint32_t* name_offsets, uint32_t unk_id, gtgpu_buf** out_ids);
+/* Tokenizer::encode(RegionSet::try_from(file f)) for a batch of n_files BED files in one device pass.  Inputs as in
+ * gtgpu_igd_count_bed / _gz: file f = text[file_offsets[f], file_offsets[f+1]) of any total size, or the gzip members
+ * [file_members[f], file_members[f+1]) of gz / member_offsets (as in gtgpu_gunzip; inflated whole into device memory,
+ * GTGPU_ERR_NOMEM when that text does not fit).  Line rules, windows of about GTGPU_INGEST_WINDOW bytes, the header rule per
+ * file and the errors are those of gtgpu_igd_build_bed (GTGPU_ERR_INVALID: a malformed line, "file k, line j", j 1-based in file
+ * k; a file without a region line, "file k: ... 0 regions found"; GTGPU_ERR_UNSUPPORTED: more than 262 144 distinct names or
+ * 2^32 - 1 region lines or more).  Chromosome names map through the caller's table as in gtgpu_tokenize_bed; a name not in it
+ * produces no hits.  Every file's regions are stable-sorted by (chromosome string, start) on the device unless every file is
+ * already in that order.  Outputs as gtgpu_tokenize_files: out_file_token_offsets (n_files + 1, caller-allocated) into *out_ids;
+ * file f's ids equal gtgpu_tokenize_bed on file f alone (hits in the backend's order, [unk_id] for a file without a token).
+ * n_files == 0 gives the offsets [0] and an empty buffer.  On a multi-device ctx the call runs on the first device. */
+int32_t gtgpu_tokenize_bed_files(gtgpu_index* index, uint64_t n_files, const char* text, const uint64_t* file_offsets,
+                                 uint32_t n_names, const char* names, const uint32_t* name_offsets, uint32_t unk_id,
+                                 uint64_t* out_file_token_offsets, gtgpu_buf** out_ids);
+int32_t gtgpu_tokenize_bed_files_gz(gtgpu_index* index, uint64_t n_files, const uint64_t* file_members, uint64_t n_members,
+                                    const uint8_t* gz, const uint64_t* member_offsets, uint32_t n_names, const char* names,
+                                    const uint32_t* name_offsets, uint32_t unk_id, uint64_t* out_file_token_offsets,
+                                    gtgpu_buf** out_ids);
 
 /* tokenize_fragment_file (gtars-tokenizers/src/utils/fragments.rs:12-82) from the file's (decompressed) text: lines
  * starting with '#' are skipped, every other line needs at least five whitespace-separated fields (chr start end
