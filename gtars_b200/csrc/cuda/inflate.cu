@@ -117,9 +117,12 @@ __device__ __forceinline__ uint64_t consumed(const Bits& b) { return b.pos - (b.
 __device__ __forceinline__ uint32_t bit_reverse(uint32_t v, uint32_t n) { return __brev(v) >> (32 - n); }
 
 // Canonical Huffman tables from code lengths (RFC 1951 3.2.2): per-length counts, symbols ordered by (length, symbol) for
-// the bit-by-bit path, and the first-level table for codes of at most FB bits.  Returns false for an over-subscribed set.
+// the bit-by-bit path, and the first-level table for codes of at most FB bits.  Returns false for an over-subscribed set and
+// for an incomplete one, except that a literal/length or distance code (`sparse`) may hold no code or a single 1-bit code:
+// the sets zlib accepts (RFC 1951 3.2.7 allows one distance code).  A bit pattern no code covers is then a decode error.
 template <int FB>
-__device__ bool build_tables(const uint8_t* len, uint32_t n, uint16_t* cnt, uint16_t* sym, uint16_t* fast, uint32_t lane) {
+__device__ bool build_tables(const uint8_t* len, uint32_t n, uint16_t* cnt, uint16_t* sym, uint16_t* fast, bool sparse,
+                             uint32_t lane) {
     __syncwarp();
     for (uint32_t i = lane; i < (1u << FB); i += 32) fast[i] = 0;
     __shared__ uint16_t s_offs_all[INF_WARPS][16];
@@ -141,6 +144,7 @@ __device__ bool build_tables(const uint8_t* len, uint32_t n, uint16_t* cnt, uint
             offs[l] = (uint16_t)o;
             o += cnt[l];
         }
+        if (left > 0 && !(sparse && (o == 0 || (o == 1 && cnt[1] == 1)))) ok = false;
         if (ok)
             for (uint32_t s = 0; s < n; ++s)
                 if (len[s]) sym[offs[len[s]]++] = (uint16_t)s;
@@ -307,8 +311,9 @@ __global__ void __launch_bounds__(INF_WARPS * 32) gunzip_kernel(uint64_t n_membe
                     for (uint32_t s = lane; s < 288; s += 32) m.len[s] = s < 144 ? 8 : s < 256 ? 9 : s < 280 ? 7 : 8;
                     for (uint32_t s = lane; s < 32; s += 32) m.len[288 + s] = 5;
                     __syncwarp();
-                    build_tables<LL_BITS>(m.len, 288, m.ll_cnt, m.ll_sym, m.ll_fast, lane);
-                    build_tables<D_BITS>(m.len + 288, 30, m.d_cnt, m.d_sym, m.d_fast, lane);
+                    build_tables<LL_BITS>(m.len, 288, m.ll_cnt, m.ll_sym, m.ll_fast, true, lane);
+                    // all 32 distance codes: a complete set (codes 30 and 31 are rejected when they are read)
+                    build_tables<D_BITS>(m.len + 288, 32, m.d_cnt, m.d_sym, m.d_fast, true, lane);
                 } else {  // dynamic codes (3.2.7)
                     const uint32_t hlit = take(m, b, gz, lane, 5) + 257, hdist = take(m, b, gz, lane, 5) + 1;
                     const uint32_t hclen = take(m, b, gz, lane, 4) + 4;
@@ -324,8 +329,12 @@ __global__ void __launch_bounds__(INF_WARPS * 32) gunzip_kernel(uint64_t n_membe
                         if (lane == 0) m.len[c_clen_order[i]] = (uint8_t)v;
                     }
                     __syncwarp();
+                    if (consumed(b) > in1) {  // the member ends inside its block header
+                        err = INF_INPUT_END;
+                        break;
+                    }
                     // the code-length code: 19 symbols, at most 7 bits — its tables borrow the distance arrays
-                    if (!build_tables<7>(m.len, 19, m.d_cnt, m.d_sym, m.d_fast, lane)) {
+                    if (!build_tables<7>(m.len, 19, m.d_cnt, m.d_sym, m.d_fast, false, lane)) {
                         err = INF_BAD_CODE;
                         break;
                     }
@@ -355,6 +364,7 @@ __global__ void __launch_bounds__(INF_WARPS * 32) gunzip_kernel(uint64_t n_membe
                             err = INF_BAD_CODE;
                         }
                         if (i + rep > hlit + hdist) err = INF_BAD_CODE;
+                        if (consumed(b) > in1) err = INF_INPUT_END;
                         if (!err) {
                             // lengths of the literal/length alphabet go to len[0 .. hlit), distances to len[288 ..)
                             for (uint32_t j = lane; j < rep; j += 32) {
@@ -369,8 +379,8 @@ __global__ void __launch_bounds__(INF_WARPS * 32) gunzip_kernel(uint64_t n_membe
                     for (uint32_t s = hlit + lane; s < 288; s += 32) m.len[s] = 0;
                     for (uint32_t s = hdist + lane; s < 32; s += 32) m.len[288 + s] = 0;
                     __syncwarp();
-                    if (m.len[256] == 0 || !build_tables<LL_BITS>(m.len, 288, m.ll_cnt, m.ll_sym, m.ll_fast, lane) ||
-                        !build_tables<D_BITS>(m.len + 288, 30, m.d_cnt, m.d_sym, m.d_fast, lane)) {
+                    if (m.len[256] == 0 || !build_tables<LL_BITS>(m.len, 288, m.ll_cnt, m.ll_sym, m.ll_fast, true, lane) ||
+                        !build_tables<D_BITS>(m.len + 288, 30, m.d_cnt, m.d_sym, m.d_fast, true, lane)) {
                         err = INF_BAD_CODE;
                         break;
                     }
