@@ -87,10 +87,6 @@ int32_t launch_build_luts(gtgpu_ctx* ctx, uint32_t n_desc, const LutDesc* d_desc
     return GTGPU_OK;
 }
 
-static int grid_for(const gtgpu_ctx* ctx, uint64_t n) {
-    return (int)std::max<uint64_t>(1, std::min<uint64_t>((n + 255) / 256, (uint64_t)ctx->sm_count * 16));
-}
-
 int32_t launch_gather_u32(gtgpu_ctx* ctx, uint64_t n, const uint32_t* d_src, const uint32_t* d_perm, uint32_t* d_out) {
     if (!n) return GTGPU_OK;
     build_gather_u32_kernel<<<grid_for(ctx, n), 256, 0, ctx->stream>>>(n, d_src, d_perm, d_out);

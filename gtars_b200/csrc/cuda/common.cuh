@@ -4,6 +4,7 @@
 #include <cuda_runtime.h>
 #include <stdint.h>
 
+#include <algorithm>
 #include <functional>
 #include <map>
 #include <memory>
@@ -188,6 +189,13 @@ struct gtgpu_ctx {
     int32_t pinned_get(size_t bytes, gtgpu::PinnedBlock* out);  // both take pinned_mu: callable with or without mu held
     void pinned_put(gtgpu::PinnedBlock b);
 };
+
+namespace gtgpu {
+// grid of a grid-stride kernel of 256-thread blocks over n items: one block per 256 items, at most 16 per SM
+inline int grid_for(const gtgpu_ctx* ctx, uint64_t n) {
+    return (int)std::max<uint64_t>(1, std::min<uint64_t>((n + 255) / 256, (uint64_t)ctx->sm_count * 16));
+}
+}  // namespace gtgpu
 
 struct gtgpu_buf {
     gtgpu_ctx* ctx = nullptr;
@@ -439,31 +447,51 @@ struct KeyTable {
     // Otherwise *out_names: the kept keys' bytes back to back (elem_size 1); *out_name_offsets: n_kept + 1 u64 offsets into them.
     int32_t finish(gtgpu_ctx* ctx, uint32_t* n_kept, BufPtr* out_names, BufPtr* out_name_offsets, BufPtr* out_spans = nullptr);
 };
-// A fragment text of any size in windows that end right after a '\n' (about GTGPU_INGEST_WINDOW bytes, default 2 GiB).  fn gets
-// each window's device bytes, its size, its byte offset in the file and the file-wide index of its first line, and returns
-// the window's line count.  Exactly one of host_text (staged through pinned memory) / dev_text (read in place) is given.
-using WindowFn = std::function<int32_t(const char* d_window, uint64_t n_bytes, uint64_t byte0, uint64_t first_line, uint32_t* n_lines)>;
-int32_t for_each_window(gtgpu_ctx* ctx, const char* host_text, const char* dev_text, uint64_t n_bytes, const std::string& who,
-                        const WindowFn& fn);
+// ---- the text input of the device parsers -------------------------------------------------------------------------------------
+// What an entry point was given: plain text (text, n_bytes), or gzip members (member k = gz[member_offsets[k], member_offsets[k + 1]),
+// as gtgpu_gunzip takes them), and for the entry points that take several files, where each file starts: file f =
+// text[file_offsets[f], file_offsets[f + 1]) or the members [file_members[f], file_members[f + 1]).  check() holds every argument
+// rule of these entry points (GTGPU_ERR_INVALID, "who: ..."); open_text_locked turns a checked input into a Text.
+struct TextIn {
+    const char* text = nullptr;
+    uint64_t n_bytes = 0;
+    const uint8_t* gz = nullptr;
+    uint64_t n_members = 0;
+    const uint64_t* member_offsets = nullptr;
+    bool is_gz = false, files = false;
+    uint64_t n_files = 0;
+    const uint64_t* file_offsets = nullptr;  // plain text of files: n_files + 1 byte offsets
+    const uint64_t* file_members = nullptr;  // gzip members of files: n_files + 1 member indices
+    static TextIn plain(const char* text, uint64_t n_bytes);
+    static TextIn plain(const char* text, uint64_t n_files, const uint64_t* file_offsets);
+    static TextIn gzip(uint64_t n_members, const uint8_t* gz, const uint64_t* member_offsets);
+    static TextIn gzip(uint64_t n_members, const uint8_t* gz, const uint64_t* member_offsets, uint64_t n_files, const uint64_t* file_members);
+    int32_t check(const std::string& who) const;
+};
+// The text a parser reads: n_bytes at `bytes`, in the caller's host memory (staged to the device by the parser) or, when on_device,
+// in device memory (inflated gzip members, read in place).  file_offsets: the files' n_files + 1 byte offsets in the text.
+struct Text {
+    const char* bytes = nullptr;
+    bool on_device = false;
+    uint64_t n_bytes = 0;
+    uint64_t n_files = 0;
+    std::vector<uint64_t> file_offsets;
+};
+// A checked TextIn as a Text: gzip members are inflated whole into device memory (scratch SC_GZ_OUT, by gunzip_locked) and the
+// files' member ranges become byte ranges of that text.  The caller holds ctx->mu.
+int32_t open_text_locked(gtgpu_ctx* ctx, const TextIn& in, const std::string& who, Text* out);
 // inflate.cu: H2D of gzip members + inflate; the text stays in scratch SC_GZ_OUT
-int32_t check_members(uint64_t n_members, const uint8_t* gz, const uint64_t* member_offsets, const char* who);
 int32_t gunzip_locked(gtgpu_ctx* ctx, uint64_t n_members, const uint8_t* gz, const uint64_t* member_offsets,
                       uint64_t* out_member_offsets, uint8_t** d_text, uint64_t* n_text);
-// gunzip_locked for a text parsed in windows afterwards: a text that does not fit in device memory is reported as such
-int32_t inflate_whole_locked(gtgpu_ctx* ctx, uint64_t n_members, const uint8_t* gz, const uint64_t* member_offsets, const std::string& who,
-                             uint8_t** d_text, uint64_t* n_text, uint64_t* out_member_offsets = nullptr);
-// The text is host_text (copied to the device here) or dev_text (already there, e.g. inflated): exactly one is non-null.
-int32_t tokenize_bed_locked(gtgpu_index* ix, const char* host_text, const char* dev_text, uint64_t n_bytes, uint32_t n_names,
-                            const char* names, const uint32_t* name_offsets, uint32_t unk_id, gtgpu_buf** out_ids);
-// Fragment tokenization of a text of any size; barcodes as names (out_names, out_name_offsets) or, with out_spans, as u32
-// (first byte, length) spans into the text (the text must then be < 4 GiB).
-int32_t tokenize_fragments_file_locked(gtgpu_index* ix, const char* host_text, const char* dev_text, uint64_t n_bytes, uint32_t n_names,
-                                       const char* names, const uint32_t* name_offsets, uint32_t unk_id, const std::string& who,
-                                       uint32_t* out_n_barcodes, BufPtr* out_names, BufPtr* out_name_offsets, BufPtr* out_spans,
-                                       BufPtr* out_barcode_offsets, BufPtr* out_ids);
 
-// The region lines of n_files BED files back to back (file f = text[file_offsets[f], file_offsets[f + 1]), any total size),
-// parsed on the device in windows: line rules of gtgpu_parse_bed per file, chromosome names discovered in first-appearance order.
+// A fragment text of any size in windows that end right after a '\n' (about GTGPU_INGEST_WINDOW bytes, default 2 GiB).  fn gets
+// each window's device bytes, its size, its byte offset in the file and the file-wide index of its first line, and returns
+// the window's line count.  Host text is staged through pinned memory, device text read in place.
+using WindowFn = std::function<int32_t(const char* d_window, uint64_t n_bytes, uint64_t byte0, uint64_t first_line, uint32_t* n_lines)>;
+int32_t for_each_window(gtgpu_ctx* ctx, const Text& t, const std::string& who, const WindowFn& fn);
+
+// The region lines of t.n_files BED files back to back (any total size), parsed on the device in windows: line rules of
+// gtgpu_parse_bed per file, chromosome names discovered in first-appearance order.
 // On success chr / start / end / file hold the n records in file order (chr = dense name id), file_offsets the files' record
 // offsets (n_files + 1), names / name_offsets the n_names chromosome names in id order.  The caller holds ctx->mu.
 struct BedFilesRecords {
@@ -473,18 +501,11 @@ struct BedFilesRecords {
     uint32_t n_names = 0;
     BufPtr names, name_offsets;
 };
-int32_t parse_bed_files_locked(gtgpu_ctx* ctx, const char* host_text, const char* dev_text, uint64_t n_files, const uint64_t* file_offsets,
-                               const std::string& who, BedFilesRecords* out);
+int32_t parse_bed_files_locked(gtgpu_ctx* ctx, const Text& t, const std::string& who, BedFilesRecords* out);
 // parse_bed_files_locked for query files: every record's chr in the ids of the caller's names (GTGPU_UNKNOWN_CHROM for a name
 // not among them).  *nt: the caller's name table in scratch SC_SET_ID (with_rank adds the names' ranks), uploaded when r->n > 0.
-int32_t parse_bed_queries_locked(gtgpu_ctx* ctx, const char* host_text, const char* dev_text, uint64_t n_files,
-                                 const uint64_t* file_offsets, uint32_t n_names, const char* names, const uint32_t* name_offsets,
+int32_t parse_bed_queries_locked(gtgpu_ctx* ctx, const Text& t, uint32_t n_names, const char* names, const uint32_t* name_offsets,
                                  bool with_rank, const std::string& who, BedFilesRecords* r, NameTable* nt);
-// gtgpu_tokenize_bed_files on text already split into n_files > 0 files (exactly one of host_text / dev_text is given):
-// out_file_token_offsets (n_files + 1, host) and *out_ids as gtgpu_tokenize_files returns them.
-int32_t tokenize_bed_files_locked(gtgpu_index* ix, const char* host_text, const char* dev_text, uint64_t n_files,
-                                  const uint64_t* file_offsets, uint32_t n_names, const char* names, const uint32_t* name_offsets,
-                                  uint32_t unk_id, const std::string& who, uint64_t* out_file_token_offsets, BufPtr* out_ids);
 
 // groups (api.cu, comm.cu, igd.cu)
 int32_t for_each_device(size_t n_devices, const std::function<int32_t(size_t)>& fn);

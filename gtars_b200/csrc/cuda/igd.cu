@@ -62,10 +62,6 @@ struct TempPool {
     }
 };
 
-int grid_for(const gtgpu_ctx* ctx, uint64_t n) {
-    return (int)std::max<uint64_t>(1, std::min<uint64_t>((n + 255) / 256, (uint64_t)ctx->sm_count * 16));
-}
-
 }  // namespace
 
 // ---- build kernels ---------------------------------------------------------------------------------------------------
@@ -421,11 +417,23 @@ extern "C" int32_t gtgpu_igd_build(gtgpu_ctx* ctx, uint64_t n_files, const uint6
 } GT_CATCH
 
 // ---- a database from its BED files' text, parsed on the device --------------------------------------------------------------
-// The records and the chromosome names come from parse_bed_files_locked on ctx (the first device of a group).  One device: the
-// build reads the parsed records where they are.  A group: shard r's files are a contiguous record range, copied to its
-// device with cudaMemcpyAsync by the builder of gtgpu_igd_build (igd_records_to_device).
-static int32_t igd_build_parsed(gtgpu_ctx* ctx, uint64_t n_files, BedFilesRecords& r, uint32_t* out_n_chroms, gtgpu_buf** out_names,
-                                gtgpu_buf** out_name_offsets, gtgpu_igd** out_igd) {
+// The records and the chromosome names come from parse_bed_files_locked on ctx (the first device of a group); ctx->mu is released
+// before the build.  One device: the build reads the parsed records where they are.  A group: shard r's files are a contiguous
+// record range, copied to its device with cudaMemcpyAsync by the builder of gtgpu_igd_build (igd_records_to_device).  The body of
+// the plain-text / gzip pair (`who`: the entry point's name without "gtgpu_").
+static int32_t igd_build_bed_text(gtgpu_ctx* ctx, const TextIn& in, const char* who, uint32_t* out_n_chroms, gtgpu_buf** out_names,
+                                  gtgpu_buf** out_name_offsets, gtgpu_igd** out_igd) {
+    if (!ctx || !out_n_chroms || !out_names || !out_name_offsets || !out_igd) return fail(GTGPU_ERR_INVALID, std::string(who) + ": null argument");
+    GT_TRY(in.check(who));
+    const uint64_t n_files = in.n_files;
+    BedFilesRecords r;
+    {
+        std::lock_guard<std::mutex> lk(ctx->mu);
+        GT_CUDA(cudaSetDevice(ctx->device));
+        Text t;
+        GT_TRY(open_text_locked(ctx, in, who, &t));
+        GT_TRY(parse_bed_files_locked(ctx, t, who, &r));
+    }
     const uint32_t n_chroms = r.n_names;
     gtgpu_igd* g = nullptr;
     if (ctx->peers.size() > 1) {
@@ -446,45 +454,15 @@ static int32_t igd_build_parsed(gtgpu_ctx* ctx, uint64_t n_files, BedFilesRecord
 extern "C" int32_t gtgpu_igd_build_bed(gtgpu_ctx* ctx, uint64_t n_files, const char* text, const uint64_t* file_offsets,
                                        uint32_t* out_n_chroms, gtgpu_buf** out_chrom_names, gtgpu_buf** out_chrom_name_offsets,
                                        gtgpu_igd** out_igd) try {
-    if (!ctx || !file_offsets || !out_n_chroms || !out_chrom_names || !out_chrom_name_offsets || !out_igd)
-        return fail(GTGPU_ERR_INVALID, "igd_build_bed: null argument");
-    if (file_offsets[0] != 0) return fail(GTGPU_ERR_INVALID, "igd_build_bed: file_offsets[0] must be 0");
-    for (uint64_t f = 0; f < n_files; ++f)
-        if (file_offsets[f] > file_offsets[f + 1]) return fail(GTGPU_ERR_INVALID, "igd_build_bed: file_offsets not monotone");
-    if (file_offsets[n_files] && !text) return fail(GTGPU_ERR_INVALID, "igd_build_bed: null text");
-    if (n_files >= 0xFFFFFFFFull) return fail(GTGPU_ERR_UNSUPPORTED, "igd_build_bed: too many files");
-    BedFilesRecords r;
-    {
-        std::lock_guard<std::mutex> lk(ctx->mu);
-        GT_CUDA(cudaSetDevice(ctx->device));
-        GT_TRY(parse_bed_files_locked(ctx, text, nullptr, n_files, file_offsets, "igd_build_bed", &r));
-    }
-    return igd_build_parsed(ctx, n_files, r, out_n_chroms, out_chrom_names, out_chrom_name_offsets, out_igd);
+    return igd_build_bed_text(ctx, TextIn::plain(text, n_files, file_offsets), "igd_build_bed", out_n_chroms, out_chrom_names,
+                              out_chrom_name_offsets, out_igd);
 } GT_CATCH
 
 extern "C" int32_t gtgpu_igd_build_bed_gz(gtgpu_ctx* ctx, uint64_t n_files, const uint64_t* file_members, uint64_t n_members,
                                           const uint8_t* gz, const uint64_t* member_offsets, uint32_t* out_n_chroms,
                                           gtgpu_buf** out_chrom_names, gtgpu_buf** out_chrom_name_offsets, gtgpu_igd** out_igd) try {
-    if (!ctx || !file_members || !out_n_chroms || !out_chrom_names || !out_chrom_name_offsets || !out_igd)
-        return fail(GTGPU_ERR_INVALID, "igd_build_bed_gz: null argument");
-    GT_TRY(check_members(n_members, gz, member_offsets, "igd_build_bed_gz"));
-    if (file_members[0] != 0 || file_members[n_files] != n_members)
-        return fail(GTGPU_ERR_INVALID, "igd_build_bed_gz: file_members must run from 0 to n_members");
-    for (uint64_t f = 0; f < n_files; ++f)
-        if (file_members[f] > file_members[f + 1]) return fail(GTGPU_ERR_INVALID, "igd_build_bed_gz: file_members not monotone");
-    if (n_files >= 0xFFFFFFFFull) return fail(GTGPU_ERR_UNSUPPORTED, "igd_build_bed_gz: too many files");
-    BedFilesRecords r;
-    {
-        std::lock_guard<std::mutex> lk(ctx->mu);
-        GT_CUDA(cudaSetDevice(ctx->device));
-        uint8_t* d_text = nullptr;
-        uint64_t n_text = 0;
-        std::vector<uint64_t> text_offsets(n_members + 1), fo(n_files + 1);
-        GT_TRY(inflate_whole_locked(ctx, n_members, gz, member_offsets, "igd_build_bed_gz", &d_text, &n_text, text_offsets.data()));
-        for (uint64_t f = 0; f <= n_files; ++f) fo[f] = text_offsets[file_members[f]];
-        GT_TRY(parse_bed_files_locked(ctx, nullptr, (const char*)d_text, n_files, fo.data(), "igd_build_bed_gz", &r));
-    }
-    return igd_build_parsed(ctx, n_files, r, out_n_chroms, out_chrom_names, out_chrom_name_offsets, out_igd);
+    return igd_build_bed_text(ctx, TextIn::gzip(n_members, gz, member_offsets, n_files, file_members), "igd_build_bed_gz", out_n_chroms,
+                              out_chrom_names, out_chrom_name_offsets, out_igd);
 } GT_CATCH
 
 // Records to the device: chr / start / end (host or device memory, any device: cudaMemcpyDefault) into temporaries of tp, and
@@ -839,83 +817,57 @@ extern "C" int32_t gtgpu_igd_count_dev(gtgpu_igd* igd, int32_t binary, uint64_t 
 } GT_CATCH
 
 // ---- query sets from their BED files' text, parsed on the device (parse_bed_queries_locked) ---------------------------------
-// The parsed query sets against g.  One device counts the columns where the parse left them; a group runs its sharded count
-// with them as query arrays (each device pulls them from the first one) and gathers the shards' columns.
-static int32_t igd_count_parsed(gtgpu_igd* g, bool binary, uint64_t n_sets, const BedFilesRecords& r, int32_t m, uint64_t* out,
-                                uint64_t* out_set_regions) {
-    gtgpu_ctx* ctx = g->ctx;
-    if (!g->shards.empty()) {
-        const int32_t s = igd_count_group(g, binary, n_sets, r.file_offsets.data(), r.chr.u32(), r.start.u32(), r.end.u32(), m, out);
+// The parsed query sets against igd; ctx->mu is released before the count.  One device counts the columns where the parse left
+// them; a group runs its sharded count with them as query arrays (each device pulls them from the first one) and gathers the
+// shards' columns.  The body of the plain-text / gzip pair (`who`: the entry point's name without "gtgpu_").
+static int32_t igd_count_bed_text(gtgpu_igd* igd, int32_t binary, const TextIn& in, const char* who, uint32_t n_names, const char* names,
+                                  const uint32_t* name_offsets, int32_t min_overlap, uint64_t* out, uint64_t* out_set_regions) {
+    if (!igd || !out || !out_set_regions || (n_names && (!names || !name_offsets)))
+        return fail(GTGPU_ERR_INVALID, std::string(who) + ": null argument");
+    const uint64_t n_sets = in.n_files;
+    if (n_sets >= 0xFFFFFFFFull) return fail(GTGPU_ERR_UNSUPPORTED, std::string(who) + ": too many sets");
+    if (min_overlap < 1)
+        return fail(GTGPU_ERR_UNSUPPORTED, std::string(who) + ": min_overlap < 1 depends on the reference's tile layout and is not supported");
+    GT_TRY(in.check(who));
+    if (n_sets == 0) return GTGPU_OK;
+    gtgpu_ctx* ctx = igd->ctx;
+    BedFilesRecords r;
+    {
+        std::lock_guard<std::mutex> lk(ctx->mu);
+        GT_CUDA(cudaSetDevice(ctx->device));
+        Text t;
+        GT_TRY(open_text_locked(ctx, in, who, &t));
+        NameTable nt;
+        GT_TRY(parse_bed_queries_locked(ctx, t, n_names, names, name_offsets, false, who, &r, &nt));
+    }
+    if (!igd->shards.empty()) {
+        const int32_t s =
+            igd_count_group(igd, binary != 0, n_sets, r.file_offsets.data(), r.chr.u32(), r.start.u32(), r.end.u32(), min_overlap, out);
         GT_CUDA(cudaSetDevice(ctx->device));  // the parsed records are freed on their device
         GT_TRY(s);
     } else {
         std::lock_guard<std::mutex> lk(ctx->mu);
         GT_CUDA(cudaSetDevice(ctx->device));
-        GT_TRY(igd_count_to_host_locked(g, binary, n_sets, r.n, r.file.u32(), r.chr.u32(), r.start.u32(), r.end.u32(), m, out));
+        GT_TRY(igd_count_to_host_locked(igd, binary != 0, n_sets, r.n, r.file.u32(), r.chr.u32(), r.start.u32(), r.end.u32(), min_overlap,
+                                        out));
     }
     for (uint64_t s = 0; s < n_sets; ++s) out_set_regions[s] = r.file_offsets[s + 1] - r.file_offsets[s];
-    return GTGPU_OK;
-}
-
-static int32_t igd_count_bed_check(const char* who, gtgpu_igd* igd, uint64_t n_sets, uint32_t n_names, const char* names,
-                                   const uint32_t* name_offsets, int32_t min_overlap, uint64_t* out, uint64_t* out_set_regions) {
-    if (!igd || !out || !out_set_regions || (n_names && (!names || !name_offsets)))
-        return fail(GTGPU_ERR_INVALID, std::string(who) + ": null argument");
-    if (n_sets >= 0xFFFFFFFFull) return fail(GTGPU_ERR_UNSUPPORTED, std::string(who) + ": too many sets");
-    if (min_overlap < 1)
-        return fail(GTGPU_ERR_UNSUPPORTED, std::string(who) + ": min_overlap < 1 depends on the reference's tile layout and is not supported");
     return GTGPU_OK;
 }
 
 extern "C" int32_t gtgpu_igd_count_bed(gtgpu_igd* igd, int32_t binary, uint64_t n_sets, const char* text, const uint64_t* file_offsets,
                                        uint32_t n_names, const char* names, const uint32_t* name_offsets, int32_t min_overlap,
                                        uint64_t* out, uint64_t* out_set_regions) try {
-    GT_TRY(igd_count_bed_check("igd_count_bed", igd, n_sets, n_names, names, name_offsets, min_overlap, out, out_set_regions));
-    if (!file_offsets) return fail(GTGPU_ERR_INVALID, "igd_count_bed: null argument");
-    if (file_offsets[0] != 0) return fail(GTGPU_ERR_INVALID, "igd_count_bed: file_offsets[0] must be 0");
-    for (uint64_t s = 0; s < n_sets; ++s)
-        if (file_offsets[s] > file_offsets[s + 1]) return fail(GTGPU_ERR_INVALID, "igd_count_bed: file_offsets not monotone");
-    if (file_offsets[n_sets] && !text) return fail(GTGPU_ERR_INVALID, "igd_count_bed: null text");
-    if (n_sets == 0) return GTGPU_OK;
-    gtgpu_ctx* ctx = igd->ctx;
-    BedFilesRecords r;
-    {
-        std::lock_guard<std::mutex> lk(ctx->mu);
-        GT_CUDA(cudaSetDevice(ctx->device));
-        NameTable nt;
-        GT_TRY(parse_bed_queries_locked(ctx, text, nullptr, n_sets, file_offsets, n_names, names, name_offsets, false, "igd_count_bed",
-                                        &r, &nt));
-    }
-    return igd_count_parsed(igd, binary != 0, n_sets, r, min_overlap, out, out_set_regions);
+    return igd_count_bed_text(igd, binary, TextIn::plain(text, n_sets, file_offsets), "igd_count_bed", n_names, names, name_offsets,
+                              min_overlap, out, out_set_regions);
 } GT_CATCH
 
 extern "C" int32_t gtgpu_igd_count_bed_gz(gtgpu_igd* igd, int32_t binary, uint64_t n_sets, const uint64_t* file_members,
                                           uint64_t n_members, const uint8_t* gz, const uint64_t* member_offsets, uint32_t n_names,
                                           const char* names, const uint32_t* name_offsets, int32_t min_overlap, uint64_t* out,
                                           uint64_t* out_set_regions) try {
-    GT_TRY(igd_count_bed_check("igd_count_bed_gz", igd, n_sets, n_names, names, name_offsets, min_overlap, out, out_set_regions));
-    if (!file_members) return fail(GTGPU_ERR_INVALID, "igd_count_bed_gz: null argument");
-    GT_TRY(check_members(n_members, gz, member_offsets, "igd_count_bed_gz"));
-    if (file_members[0] != 0 || file_members[n_sets] != n_members)
-        return fail(GTGPU_ERR_INVALID, "igd_count_bed_gz: file_members must run from 0 to n_members");
-    for (uint64_t s = 0; s < n_sets; ++s)
-        if (file_members[s] > file_members[s + 1]) return fail(GTGPU_ERR_INVALID, "igd_count_bed_gz: file_members not monotone");
-    if (n_sets == 0) return GTGPU_OK;
-    gtgpu_ctx* ctx = igd->ctx;
-    BedFilesRecords r;
-    {
-        std::lock_guard<std::mutex> lk(ctx->mu);
-        GT_CUDA(cudaSetDevice(ctx->device));
-        uint8_t* d_text = nullptr;
-        uint64_t n_text = 0;
-        std::vector<uint64_t> text_offsets(n_members + 1), fo(n_sets + 1);
-        GT_TRY(inflate_whole_locked(ctx, n_members, gz, member_offsets, "igd_count_bed_gz", &d_text, &n_text, text_offsets.data()));
-        for (uint64_t s = 0; s <= n_sets; ++s) fo[s] = text_offsets[file_members[s]];
-        NameTable nt;
-        GT_TRY(parse_bed_queries_locked(ctx, nullptr, (const char*)d_text, n_sets, fo.data(), n_names, names, name_offsets, false,
-                                        "igd_count_bed_gz", &r, &nt));
-    }
-    return igd_count_parsed(igd, binary != 0, n_sets, r, min_overlap, out, out_set_regions);
+    return igd_count_bed_text(igd, binary, TextIn::gzip(n_members, gz, member_offsets, n_sets, file_members), "igd_count_bed_gz", n_names,
+                              names, name_offsets, min_overlap, out, out_set_regions);
 } GT_CATCH
 
 // ---- .igd bytes of a database, written from the device -----------------------------------------------------------------------

@@ -622,20 +622,82 @@ int32_t gunzip_locked(gtgpu_ctx* ctx, uint64_t n_members, const uint8_t* gz, con
     return gunzip_device(ctx, n_members, d_gz, d_mo, d_oo, d_out, d_status, h_status);
 }
 
-// gzip members -> device text (SC_GZ_OUT); a text that does not fit in device memory is reported as such
-int32_t inflate_whole_locked(gtgpu_ctx* ctx, uint64_t n_members, const uint8_t* gz, const uint64_t* member_offsets, const std::string& who,
-                             uint8_t** d_text, uint64_t* n_text, uint64_t* out_member_offsets) {
-    const int32_t s = gunzip_locked(ctx, n_members, gz, member_offsets, out_member_offsets, d_text, n_text);
+TextIn TextIn::plain(const char* text, uint64_t n_bytes) {
+    TextIn in;
+    in.text = text;
+    in.n_bytes = n_bytes;
+    return in;
+}
+
+TextIn TextIn::plain(const char* text, uint64_t n_files, const uint64_t* file_offsets) {
+    TextIn in;
+    in.text = text;
+    in.files = true;
+    in.n_files = n_files;
+    in.file_offsets = file_offsets;
+    return in;
+}
+
+TextIn TextIn::gzip(uint64_t n_members, const uint8_t* gz, const uint64_t* member_offsets) {
+    TextIn in;
+    in.is_gz = true;
+    in.n_members = n_members;
+    in.gz = gz;
+    in.member_offsets = member_offsets;
+    return in;
+}
+
+TextIn TextIn::gzip(uint64_t n_members, const uint8_t* gz, const uint64_t* member_offsets, uint64_t n_files, const uint64_t* file_members) {
+    TextIn in = gzip(n_members, gz, member_offsets);
+    in.files = true;
+    in.n_files = n_files;
+    in.file_members = file_members;
+    return in;
+}
+
+int32_t TextIn::check(const std::string& who) const {
+    auto invalid = [&](const char* what) { return fail(GTGPU_ERR_INVALID, who + ": " + what); };
+    if (is_gz) {
+        if ((n_members && (!gz || !member_offsets)) || (files && !file_members)) return invalid("null argument");
+        for (uint64_t k = 0; k < n_members; ++k)
+            if (member_offsets[k] > member_offsets[k + 1]) return invalid("member_offsets not monotone");
+        if (!files) return GTGPU_OK;
+        if (file_members[0] != 0 || file_members[n_files] != n_members) return invalid("file_members must run from 0 to n_members");
+        for (uint64_t f = 0; f < n_files; ++f)
+            if (file_members[f] > file_members[f + 1]) return invalid("file_members not monotone");
+    } else if (!files) {
+        return n_bytes && !text ? invalid("null argument") : GTGPU_OK;
+    } else {
+        if (!file_offsets) return invalid("null argument");
+        if (file_offsets[0] != 0) return invalid("file_offsets[0] must be 0");
+        for (uint64_t f = 0; f < n_files; ++f)
+            if (file_offsets[f] > file_offsets[f + 1]) return invalid("file_offsets not monotone");
+        if (file_offsets[n_files] && !text) return invalid("null text");
+    }
+    if (n_files >= 0xFFFFFFFFull) return fail(GTGPU_ERR_UNSUPPORTED, who + ": too many files");
+    return GTGPU_OK;
+}
+
+int32_t open_text_locked(gtgpu_ctx* ctx, const TextIn& in, const std::string& who, Text* out) {
+    out->n_files = in.n_files;
+    if (!in.is_gz) {
+        out->bytes = in.text;
+        out->on_device = false;
+        out->n_bytes = in.files ? in.file_offsets[in.n_files] : in.n_bytes;
+        if (in.files) out->file_offsets.assign(in.file_offsets, in.file_offsets + in.n_files + 1);
+        return GTGPU_OK;
+    }
+    std::vector<uint64_t> text_offsets(in.n_members + 1);
+    uint8_t* d_text = nullptr;
+    const int32_t s = gunzip_locked(ctx, in.n_members, in.gz, in.member_offsets, text_offsets.data(), &d_text, &out->n_bytes);
     if (s == GTGPU_ERR_NOMEM)
         return fail(s, who + ": the inflated text does not fit in device memory (gzip input is inflated whole before it is parsed): " +
                            gtgpu_last_error());
-    return s;
-}
-
-int32_t check_members(uint64_t n_members, const uint8_t* gz, const uint64_t* member_offsets, const char* who) {
-    if (n_members && (!gz || !member_offsets)) return fail(GTGPU_ERR_INVALID, std::string(who) + ": null argument");
-    for (uint64_t k = 0; k < n_members; ++k)
-        if (member_offsets[k] > member_offsets[k + 1]) return fail(GTGPU_ERR_INVALID, std::string(who) + ": member_offsets not monotone");
+    GT_TRY(s);
+    out->bytes = (const char*)d_text;
+    out->on_device = true;
+    if (in.files)
+        for (uint64_t f = 0; f <= in.n_files; ++f) out->file_offsets.push_back(text_offsets[in.file_members[f]]);
     return GTGPU_OK;
 }
 
@@ -644,7 +706,7 @@ int32_t check_members(uint64_t n_members, const uint8_t* gz, const uint64_t* mem
 extern "C" int32_t gtgpu_gunzip(gtgpu_ctx* ctx, uint64_t n_members, const uint8_t* gz, const uint64_t* member_offsets,
                                 gtgpu_buf** out_text, uint64_t* out_member_offsets) try {
     if (!ctx || !out_text || !out_member_offsets) return fail(GTGPU_ERR_INVALID, "gunzip: null argument");
-    GT_TRY(check_members(n_members, gz, member_offsets, "gunzip"));
+    GT_TRY(TextIn::gzip(n_members, gz, member_offsets).check("gunzip"));
     std::lock_guard<std::mutex> lk(ctx->mu);
     GT_CUDA(cudaSetDevice(ctx->device));
     uint8_t* d_text = nullptr;
@@ -657,86 +719,5 @@ extern "C" int32_t gtgpu_gunzip(gtgpu_ctx* ctx, uint64_t n_members, const uint8_
     const cudaError_t e = cudaStreamSynchronize(ctx->stream);
     if (e != cudaSuccess) return fail(GTGPU_ERR_CUDA, std::string("gunzip: D2H: ") + cudaGetErrorString(e));
     *out_text = buf.release();
-    return GTGPU_OK;
-} GT_CATCH
-
-// gtgpu_tokenize_bed on gzip members: inflate on the device, parse + sort + tokenize the text where it is.
-extern "C" int32_t gtgpu_tokenize_bed_gz(gtgpu_index* ix, uint64_t n_members, const uint8_t* gz, const uint64_t* member_offsets,
-                                         uint32_t n_names, const char* names, const uint32_t* name_offsets, uint32_t unk_id,
-                                         gtgpu_buf** out_ids) try {
-    if (!ix || !out_ids || (n_names && (!names || !name_offsets))) return fail(GTGPU_ERR_INVALID, "tokenize_bed_gz: null argument");
-    GT_TRY(check_members(n_members, gz, member_offsets, "tokenize_bed_gz"));
-    gtgpu_ctx* ctx = ix->ctx;
-    std::lock_guard<std::mutex> lk(ctx->mu);
-    GT_CUDA(cudaSetDevice(ctx->device));
-    uint8_t* d_text = nullptr;
-    uint64_t n_text = 0;
-    GT_TRY(gunzip_locked(ctx, n_members, gz, member_offsets, nullptr, &d_text, &n_text));
-    return tokenize_bed_locked(ix, nullptr, (const char*)d_text, n_text, n_names, names, name_offsets, unk_id, out_ids);
-} GT_CATCH
-
-// gtgpu_tokenize_fragments_text on gzip members (a bgzip'ed fragment file: thousands of members).  *out_text returns the
-// inflated text as well: the barcode spans index into it.  Errors carry the text form's name and messages.
-extern "C" int32_t gtgpu_tokenize_fragments_gz(gtgpu_index* ix, uint64_t n_members, const uint8_t* gz, const uint64_t* member_offsets,
-                                               uint32_t n_names, const char* names, const uint32_t* name_offsets, uint32_t unk_id,
-                                               uint32_t* out_n_barcodes, gtgpu_buf** out_barcode_spans,
-                                               gtgpu_buf** out_barcode_offsets, gtgpu_buf** out_ids, gtgpu_buf** out_text) try {
-    if (!ix || !out_n_barcodes || !out_barcode_spans || !out_barcode_offsets || !out_ids || !out_text ||
-        (n_names && (!names || !name_offsets)))
-        return fail(GTGPU_ERR_INVALID, "tokenize_fragments_gz: null argument");
-    GT_TRY(check_members(n_members, gz, member_offsets, "tokenize_fragments_gz"));
-    gtgpu_ctx* ctx = ix->ctx;
-    std::lock_guard<std::mutex> lk(ctx->mu);
-    GT_CUDA(cudaSetDevice(ctx->device));
-    uint8_t* d_text = nullptr;
-    uint64_t n_text = 0;
-    GT_TRY(gunzip_locked(ctx, n_members, gz, member_offsets, nullptr, &d_text, &n_text));
-    if (n_text >= 0xFFFFFFF0ull) return fail(GTGPU_ERR_UNSUPPORTED, "tokenize_fragments_text: at most 4 GiB of text per call");
-    BufPtr text, spans, offs, ids;  // the text's copy on copy_out overlaps the parse
-    int32_t s = buf_from_device(ctx, d_text, n_text, 1, ctx->copy_out, &text);
-    if (s == GTGPU_ERR_CUDA) return fail(s, "tokenize_fragments_gz: D2H of the text failed");
-    GT_TRY(s);
-    try {
-        s = tokenize_fragments_file_locked(ix, nullptr, (const char*)d_text, n_text, n_names, names, name_offsets, unk_id,
-                                           "tokenize_fragments_text", out_n_barcodes, nullptr, nullptr, &spans, &offs, &ids);
-    } catch (...) {
-        cudaStreamSynchronize(ctx->copy_out);  // the text's copy ends before its block goes back to the cache
-        throw;
-    }
-    if (s == GTGPU_OK && cudaStreamSynchronize(ctx->copy_out) != cudaSuccess) s = fail(GTGPU_ERR_CUDA, "tokenize_fragments_gz: D2H of the text failed");
-    if (s != GTGPU_OK) {
-        cudaStreamSynchronize(ctx->copy_out);
-        return s;
-    }
-    *out_barcode_spans = spans.release();
-    *out_barcode_offsets = offs.release();
-    *out_ids = ids.release();
-    *out_text = text.release();
-    return GTGPU_OK;
-} GT_CATCH
-
-// gtgpu_tokenize_fragments_file on gzip members: inflated whole into device memory, then tokenized in windows where it is.
-extern "C" int32_t gtgpu_tokenize_fragments_file_gz(gtgpu_index* ix, uint64_t n_members, const uint8_t* gz, const uint64_t* member_offsets,
-                                                    uint32_t n_names, const char* names, const uint32_t* name_offsets, uint32_t unk_id,
-                                                    uint32_t* out_n_barcodes, gtgpu_buf** out_barcode_names,
-                                                    gtgpu_buf** out_barcode_name_offsets, gtgpu_buf** out_barcode_offsets,
-                                                    gtgpu_buf** out_ids) try {
-    if (!ix || !out_n_barcodes || !out_barcode_names || !out_barcode_name_offsets || !out_barcode_offsets || !out_ids ||
-        (n_names && (!names || !name_offsets)))
-        return fail(GTGPU_ERR_INVALID, "tokenize_fragments_file_gz: null argument");
-    GT_TRY(check_members(n_members, gz, member_offsets, "tokenize_fragments_file_gz"));
-    gtgpu_ctx* ctx = ix->ctx;
-    std::lock_guard<std::mutex> lk(ctx->mu);
-    GT_CUDA(cudaSetDevice(ctx->device));
-    uint8_t* d_text = nullptr;
-    uint64_t n_text = 0;
-    GT_TRY(inflate_whole_locked(ctx, n_members, gz, member_offsets, "tokenize_fragments_file_gz", &d_text, &n_text));
-    BufPtr nm, no, offs, ids;
-    GT_TRY(tokenize_fragments_file_locked(ix, nullptr, (const char*)d_text, n_text, n_names, names, name_offsets, unk_id,
-                                          "tokenize_fragments_file_gz", out_n_barcodes, &nm, &no, nullptr, &offs, &ids));
-    *out_barcode_names = nm.release();
-    *out_barcode_name_offsets = no.release();
-    *out_barcode_offsets = offs.release();
-    *out_ids = ids.release();
     return GTGPU_OK;
 } GT_CATCH

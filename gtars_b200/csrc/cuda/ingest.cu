@@ -464,10 +464,6 @@ __global__ void ingest_key_ids_kernel(uint64_t n, const uint32_t* __restrict__ k
     }
 }
 
-static int igrid(gtgpu_ctx* ctx, uint64_t n) {
-    return (int)std::max<uint64_t>(1, std::min<uint64_t>((n + 255) / 256, (uint64_t)ctx->sm_count * 16));
-}
-
 // Name table in scratch SC_SET_ID: FNV-1a hashes of the caller's chromosome names, sorted for the device lookup, and (with_rank)
 // the names' lexicographic ranks for the sort of gtgpu_parse_bed.
 int32_t upload_name_table(gtgpu_ctx* ctx, uint32_t n_names, const char* names, const uint32_t* name_offsets, NameTable* out,
@@ -519,7 +515,7 @@ static int32_t line_breaks_locked(gtgpu_ctx* ctx, const char* d_text, uint64_t n
     GT_TRY(ctx->scratch_get(SC_COUNTS, n_chunks * 4 + 4, (void**)&d_counts));
     GT_TRY(ctx->scratch_get(SC_IN3_CHR, n_chunks * 4 + 4, (void**)&d_crank));
     GT_TRY(ctx->scratch_get(SC_IN3_START, exclusive_scan_temp_bytes(n_chunks, 4), &d_tmp));
-    ingest_count_newlines_kernel<<<igrid(ctx, n_chunks), 256, 0, st>>>(n_bytes, d_text, d_counts, d_fstart, n_fstart);
+    ingest_count_newlines_kernel<<<grid_for(ctx, n_chunks), 256, 0, st>>>(n_bytes, d_text, d_counts, d_fstart, n_fstart);
     ctx->launches++;
     GT_TRY(exclusive_scan<uint32_t>(ctx, d_counts, d_crank, n_chunks, d_tmp));
     uint32_t last[2];
@@ -531,7 +527,7 @@ static int32_t line_breaks_locked(gtgpu_ctx* ctx, const char* d_text, uint64_t n
     *n_breaks = last[0] + last[1];
     *n_lines = *n_breaks + (last_byte != '\n' ? 1u : 0u);
     GT_TRY(ctx->scratch_get(SC_IN3_END, (size_t)*n_breaks * 4 + 4, (void**)d_nl));
-    ingest_newline_positions_kernel<<<igrid(ctx, n_chunks), 256, 0, st>>>(n_bytes, d_text, d_crank, *d_nl, d_fstart, n_fstart);
+    ingest_newline_positions_kernel<<<grid_for(ctx, n_chunks), 256, 0, st>>>(n_bytes, d_text, d_crank, *d_nl, d_fstart, n_fstart);
     ctx->launches++;
     return GTGPU_OK;
 }
@@ -569,7 +565,7 @@ int32_t parse_lines_locked(gtgpu_ctx* ctx, const char* d_text, uint64_t n_bytes,
     uint32_t* d_flags = reinterpret_cast<uint32_t*>(d_misc);  // [0] first malformed line, [1..3] for the caller
     const uint32_t init[4] = {0xFFFFFFFFu, 0u, 0u, 0u};
     GT_CUDA(cudaMemcpyAsync(d_flags, init, 16, cudaMemcpyHostToDevice, st));
-    const int grid = igrid(ctx, n_lines);
+    const int grid = grid_for(ctx, n_lines);
     switch (fmt) {
     case BED_LINES:
         ingest_parse_lines_kernel<false><<<grid, 256, 0, st>>>(n_lines, n_breaks, n_bytes, d_text, d_nl, nt, p, d_flags, files);
@@ -646,9 +642,10 @@ struct StagingScope {  // pinned staging blocks and their events, returned to th
     }
 };
 
-int32_t for_each_window(gtgpu_ctx* ctx, const char* host_text, const char* dev_text, uint64_t n_bytes, const std::string& who,
-                        const WindowFn& fn) {
+int32_t for_each_window(gtgpu_ctx* ctx, const Text& t, const std::string& who, const WindowFn& fn) {
     cudaStream_t st = ctx->stream;
+    const uint64_t n_bytes = t.n_bytes;
+    const char *host_text = t.on_device ? nullptr : t.bytes, *dev_text = t.on_device ? t.bytes : nullptr;
     const uint64_t W = ingest_window_bytes();
     std::vector<uint64_t> cut{0};  // window w = [cut[w], cut[w + 1])
     while (cut.back() < n_bytes) {
@@ -734,21 +731,71 @@ int32_t for_each_window(gtgpu_ctx* ctx, const char* host_text, const char* dev_t
     return GTGPU_OK;
 }
 
+// RegionSet::sort (region_set.rs:502-505) of n parsed records: stable by (chromosome rank, start), within each file when `file` (the
+// records' file indices, in file order) is given.  When some pair is out of order: stable radix passes by start, then by rank (the
+// file index folded above it when both fit 32 bits, else one more pass by file), and a gather.  The sorted columns replace *chr /
+// *start / *end; they lie in scratch SC_ING_0..3, which the fused find after the sort does not touch.  The caller holds ctx->mu.
+static int32_t sort_regions_locked(gtgpu_ctx* ctx, uint32_t n, const NameTable& nt, uint32_t n_names, const uint32_t* file,
+                                   uint64_t n_files, const uint32_t** chr, const uint32_t** start, const uint32_t** end) {
+    cudaStream_t st = ctx->stream;
+    uint32_t* d_flag;
+    GT_TRY(ctx->scratch_get(SC_MISC, 64, (void**)&d_flag));
+    GT_CUDA(cudaMemsetAsync(d_flag, 0, 4, st));
+    ingest_check_sorted_kernel<<<grid_for(ctx, n), 256, 0, st>>>(n, *chr, *start, nt.rank, n_names, d_flag, file);
+    ctx->launches++;
+    uint32_t unsorted = 0;
+    GT_CUDA(cudaMemcpyAsync(&unsorted, d_flag, 4, cudaMemcpyDeviceToHost, st));
+    GT_CUDA(cudaStreamSynchronize(st));
+    GT_CUDA(cudaGetLastError());
+    if (!unsorted) return GTGPU_OK;
+    uint32_t *k_a, *v_a, *k_b, *v_b;
+    void* d_tmp;
+    GT_TRY(ctx->scratch_get(SC_ING_0, (size_t)n * 4, (void**)&k_a));
+    GT_TRY(ctx->scratch_get(SC_ING_1, (size_t)n * 4, (void**)&v_a));
+    GT_TRY(ctx->scratch_get(SC_ING_2, (size_t)n * 4, (void**)&k_b));
+    GT_TRY(ctx->scratch_get(SC_ING_3, (size_t)n * 4, (void**)&v_b));
+    GT_TRY(ctx->scratch_get(SC_IN3_START, radix_sort_temp_bytes(n), &d_tmp));
+    GT_CUDA(cudaMemcpyAsync(k_a, *start, (size_t)n * 4, cudaMemcpyDeviceToDevice, st));
+    ingest_iota_kernel<<<grid_for(ctx, n), 256, 0, st>>>(n, v_a);
+    ctx->launches++;
+    int in_b = 0;
+    GT_TRY(radix_sort_pairs(ctx, n, k_a, v_a, k_b, v_b, 32, d_tmp, &in_b));
+    if (in_b) { std::swap(k_a, k_b); std::swap(v_a, v_b); }
+    const int rank_bits = bits_for_value(n_names), file_bits = file ? bits_for_value(n_files - 1) : 0;
+    const bool fold = file && rank_bits + file_bits <= 32;
+    ingest_rank_keys_kernel<<<grid_for(ctx, n), 256, 0, st>>>(n, v_a, *chr, nt.rank, n_names, k_a, fold ? file : nullptr, rank_bits);
+    ctx->launches++;
+    GT_TRY(radix_sort_pairs(ctx, n, k_a, v_a, k_b, v_b, fold ? rank_bits + file_bits : rank_bits, d_tmp, &in_b));
+    if (in_b) { std::swap(k_a, k_b); std::swap(v_a, v_b); }
+    if (file && !fold) {
+        GT_TRY(launch_gather_u32(ctx, n, file, v_a, k_a));
+        GT_TRY(radix_sort_pairs(ctx, n, k_a, v_a, k_b, v_b, file_bits, d_tmp, &in_b));
+        if (in_b) { std::swap(k_a, k_b); std::swap(v_a, v_b); }
+    }
+    // the order is v_a; the other three buffers take the sorted columns
+    ingest_gather_kernel<<<grid_for(ctx, n), 256, 0, st>>>(n, v_a, *chr, *start, *end, k_a, k_b, v_b);
+    ctx->launches++;
+    *chr = k_a;
+    *start = k_b;
+    *end = v_b;
+    GT_CUDA(cudaGetLastError());
+    return GTGPU_OK;
+}
+
 // Parses and sorts on the device.  On success *d_chr / *d_start / *d_end point at n_out regions in device scratch
-// (valid until the next call on this ctx).  Exactly one of host_text / dev_text is given.  The caller holds ctx->mu.
-static int32_t parse_bed_locked(gtgpu_ctx* ctx, const char* host_text, const char* dev_text, uint64_t n_bytes, uint32_t n_names,
-                                const char* names, const uint32_t* name_offsets, uint64_t* n_out, uint32_t** d_chr,
-                                uint32_t** d_start, uint32_t** d_end) {
+// (valid until the next call on this ctx).  The caller holds ctx->mu.
+static int32_t parse_bed_locked(gtgpu_ctx* ctx, const Text& t, uint32_t n_names, const char* names, const uint32_t* name_offsets,
+                                uint64_t* n_out, const uint32_t** d_chr, const uint32_t** d_start, const uint32_t** d_end) {
+    const uint64_t n_bytes = t.n_bytes;
     if (n_bytes >= 0xFFFFFFF0ull) return fail(GTGPU_ERR_UNSUPPORTED, "parse_bed: at most 4 GiB of text per call (split at a line boundary)");
     if (n_names >= 0x7FFFFFFFu) return fail(GTGPU_ERR_INVALID, "parse_bed: too many chromosome names");
-    cudaStream_t st = ctx->stream;
     *n_out = 0;
     if (n_bytes == 0) return fail(GTGPU_ERR_INVALID, "parse_bed: EmptyRegionSet (no regions in the text)");
 
-    const char* d_text = dev_text;
-    if (!dev_text) {
+    const char* d_text = t.bytes;
+    if (!t.on_device) {
         GT_TRY(ctx->scratch_get(SC_OUT_IDS2, n_bytes + 64, (void**)&d_text));
-        GT_CUDA(cudaMemcpyAsync((char*)d_text, host_text, n_bytes, cudaMemcpyHostToDevice, st));
+        GT_CUDA(cudaMemcpyAsync((char*)d_text, t.bytes, n_bytes, cudaMemcpyHostToDevice, ctx->stream));
     }
     NameTable nt;
     GT_TRY(upload_name_table(ctx, n_names, names, name_offsets, &nt, true));  // synchronises: the host's text may be reused after it
@@ -756,42 +803,12 @@ static int32_t parse_bed_locked(gtgpu_ctx* ctx, const char* host_text, const cha
     GT_TRY(parse_lines_locked(ctx, d_text, n_bytes, BED_LINES, nt, BedFilesView{}, &pl));
     if (pl.bad_line != 0xFFFFFFFFu)
         return fail(GTGPU_ERR_INVALID, "parse_bed: RegionParseError: cannot parse start / end position on line " + std::to_string((uint64_t)pl.bad_line + 1));
-    const uint32_t n = pl.n;
-    if (n == 0) return fail(GTGPU_ERR_INVALID, "parse_bed: EmptyRegionSet (no regions in the text)");
-    uint32_t *o_chr = pl.chr, *o_start = pl.start, *o_end = pl.end, *d_flags = pl.flags, flags[2];
-
-    // ---- 4. RegionSet::sort: stable by (chromosome string, start) -----------------------------------------------------------
-    ingest_check_sorted_kernel<<<igrid(ctx, n), 256, 0, st>>>(n, o_chr, o_start, nt.rank, n_names, d_flags + 1);
-    ctx->launches++;
-    GT_CUDA(cudaMemcpyAsync(flags, d_flags, 8, cudaMemcpyDeviceToHost, st));
-    GT_CUDA(cudaStreamSynchronize(st));
-    if (flags[1]) {
-        uint32_t *k_a = pl.free[0], *v_a = pl.free[1], *k_b, *v_b, *g_chr = pl.free[2], *g_start = pl.free[3], *g_end = pl.free[4];
-        void* d_tmp;
-        GT_TRY(ctx->scratch_get(SC_OUT_IDS, (size_t)n * 8 + 8, (void**)&k_b));
-        GT_TRY(ctx->scratch_get(SC_IN3_START, radix_sort_temp_bytes(n), &d_tmp));
-        v_b = k_b + n;
-        GT_CUDA(cudaMemcpyAsync(k_a, o_start, (size_t)n * 4, cudaMemcpyDeviceToDevice, st));
-        ingest_iota_kernel<<<igrid(ctx, n), 256, 0, st>>>(n, v_a);
-        ctx->launches++;
-        int in_b = 0;
-        GT_TRY(radix_sort_pairs(ctx, n, k_a, v_a, k_b, v_b, 32, d_tmp, &in_b));
-        if (in_b) { std::swap(k_a, k_b); std::swap(v_a, v_b); }
-        ingest_rank_keys_kernel<<<igrid(ctx, n), 256, 0, st>>>(n, v_a, o_chr, nt.rank, n_names, k_a);
-        ctx->launches++;
-        int bits = 1;
-        while (bits < 32 && (1ull << bits) < (uint64_t)n_names + 1) ++bits;
-        GT_TRY(radix_sort_pairs(ctx, n, k_a, v_a, k_b, v_b, bits, d_tmp, &in_b));
-        const uint32_t* order = in_b ? v_b : v_a;
-        ingest_gather_kernel<<<igrid(ctx, n), 256, 0, st>>>(n, order, o_chr, o_start, o_end, g_chr, g_start, g_end);
-        ctx->launches++;
-        o_chr = g_chr; o_start = g_start; o_end = g_end;
-    }
-    GT_CUDA(cudaGetLastError());
-    *n_out = n;
-    *d_chr = o_chr;
-    *d_start = o_start;
-    *d_end = o_end;
+    if (pl.n == 0) return fail(GTGPU_ERR_INVALID, "parse_bed: EmptyRegionSet (no regions in the text)");
+    *d_chr = pl.chr;
+    *d_start = pl.start;
+    *d_end = pl.end;
+    GT_TRY(sort_regions_locked(ctx, pl.n, nt, n_names, nullptr, 0, d_chr, d_start, d_end));
+    *n_out = pl.n;
     return GTGPU_OK;
 }
 
@@ -849,7 +866,7 @@ int32_t KeyTable::add_window(gtgpu_ctx* ctx, const char* d_text, uint64_t byte0,
         GT_CUDA(cudaMemsetAsync(t_hash.ptr, 0, new_cap * 8, st));
         GT_CUDA(cudaMemsetAsync(t_first.ptr, 0xFF, new_cap * 4, st));
         if (cap) {
-            ingest_key_rehash_kernel<<<igrid(ctx, cap), 256, 0, st>>>(cap, key_slots(hash, soff, first_byte, first, klen, known),
+            ingest_key_rehash_kernel<<<grid_for(ctx, cap), 256, 0, st>>>(cap, key_slots(hash, soff, first_byte, first, klen, known),
                                                                      (uint32_t)(new_cap - 1),
                                                                      key_slots(t_hash, t_soff, t_first_byte, t_first, t_klen, t_known));
             ctx->launches++;
@@ -865,9 +882,9 @@ int32_t KeyTable::add_window(gtgpu_ctx* ctx, const char* d_text, uint64_t byte0,
     }
     const uint32_t mask = (uint32_t)(cap - 1);
     uint32_t *slot_of = pl.free[0], *wpos = pl.free[1], *wlen = pl.free[2];
-    ingest_key_insert_kernel<<<igrid(ctx, nw), 256, 0, st>>>(nw, pl.h, mask, (unsigned long long*)hash.ptr, first.u32(), slot_of, base,
+    ingest_key_insert_kernel<<<grid_for(ctx, nw), 256, 0, st>>>(nw, pl.h, mask, (unsigned long long*)hash.ptr, first.u32(), slot_of, base,
                                                              pl.flags + 3);
-    ingest_key_heads_kernel<<<igrid(ctx, nw), 256, 0, st>>>(nw, base, slot_of, first.u32(), pl.chr, pl.bl, n_names, mask, id.u32(),
+    ingest_key_heads_kernel<<<grid_for(ctx, nw), 256, 0, st>>>(nw, base, slot_of, first.u32(), pl.chr, pl.bl, n_names, mask, id.u32(),
                                                             klen.u32(), known.u32(), wlen, pl.flags + 2);
     ctx->launches += 2;
     GT_TRY(exclusive_scan<uint32_t>(ctx, wlen, wpos, nw, pl.tmp));
@@ -880,10 +897,10 @@ int32_t KeyTable::add_window(gtgpu_ctx* ctx, const char* d_text, uint64_t byte0,
         return fail(GTGPU_ERR_UNSUPPORTED, who + ": more than " + std::to_string(max_keys) + " distinct " + keys);
     const uint64_t bytes = (uint64_t)tail[0] + tail[1];
     GT_TRY(arena.reserve(used + bytes + 1, used, st));
-    ingest_key_claim_kernel<<<igrid(ctx, nw), 256, 0, st>>>(nw, base, d_text, slot_of, id.u32(), pl.bo, pl.bl, wpos, used,
+    ingest_key_claim_kernel<<<grid_for(ctx, nw), 256, 0, st>>>(nw, base, d_text, slot_of, id.u32(), pl.bo, pl.bl, wpos, used,
                                                             (char*)arena.ptr, (unsigned long long*)soff.ptr, byte0,
                                                             (unsigned long long*)first_byte.ptr);
-    ingest_key_check_kernel<<<igrid(ctx, nw), 256, 0, st>>>(nw, base, d_text, slot_of, id.u32(), pl.bo, pl.bl, klen.u32(),
+    ingest_key_check_kernel<<<grid_for(ctx, nw), 256, 0, st>>>(nw, base, d_text, slot_of, id.u32(), pl.bo, pl.bl, klen.u32(),
                                                             (const char*)arena.ptr, (const unsigned long long*)soff.ptr, pl.flags + 1);
     ctx->launches += 2;
     uint32_t collision = 0;
@@ -913,16 +930,15 @@ int32_t KeyTable::finish(gtgpu_ctx* ctx, uint32_t* n_kept, BufPtr* out_names, Bu
         GT_TRY(ctx->scratch_get(SC_ING_3, distinct * 4, (void**)&v_b));
         GT_TRY(ctx->scratch_get(SC_MISC, 64, (void**)&d_cnt));
         GT_CUDA(cudaMemsetAsync(d_cnt, 0, 4, st));
-        ingest_key_kept_kernel<<<igrid(ctx, cap), 256, 0, st>>>(cap, (const unsigned long long*)hash.ptr, first.u32(), known.u32(), k_a,
+        ingest_key_kept_kernel<<<grid_for(ctx, cap), 256, 0, st>>>(cap, (const unsigned long long*)hash.ptr, first.u32(), known.u32(), k_a,
                                                                 v_a, d_cnt);
         ctx->launches++;
         GT_CUDA(cudaMemcpyAsync(&kept, d_cnt, 4, cudaMemcpyDeviceToHost, st));
         GT_CUDA(cudaStreamSynchronize(st));
         GT_TRY(ctx->scratch_get(SC_IN3_START, std::max(radix_sort_temp_bytes(kept), exclusive_scan_temp_bytes(kept, 8)), &d_tmp));
         if (kept) {
-            int bits = 1, in_b = 0;
-            while (bits < 32 && (1ull << bits) < n) ++bits;
-            GT_TRY(radix_sort_pairs(ctx, kept, k_a, v_a, k_b, v_b, bits, d_tmp, &in_b));
+            int in_b = 0;
+            GT_TRY(radix_sort_pairs(ctx, kept, k_a, v_a, k_b, v_b, bits_for_value(n - 1), d_tmp, &in_b));
             if (in_b) { std::swap(k_a, k_b); std::swap(v_a, v_b); }
             unsigned long long* d_len = nullptr;
             if (out_spans) {
@@ -931,7 +947,7 @@ int32_t KeyTable::finish(gtgpu_ctx* ctx, uint32_t* n_kept, BufPtr* out_names, Bu
                 GT_TRY(ctx->scratch_get(SC_ING_4, (uint64_t)kept * 8, (void**)&d_len));
                 GT_TRY(ctx->scratch_get(SC_ING_7, ((uint64_t)kept + 1) * 8, (void**)&d_noff));
             }
-            ingest_key_lengths_kernel<<<igrid(ctx, kept), 256, 0, st>>>(kept, v_a, klen.u32(), (const unsigned long long*)first_byte.ptr,
+            ingest_key_lengths_kernel<<<grid_for(ctx, kept), 256, 0, st>>>(kept, v_a, klen.u32(), (const unsigned long long*)first_byte.ptr,
                                                                         d_len, d_spans);
             ctx->launches++;
             if (!out_spans) {
@@ -942,12 +958,12 @@ int32_t KeyTable::finish(gtgpu_ctx* ctx, uint32_t* n_kept, BufPtr* out_names, Bu
                 GT_CUDA(cudaStreamSynchronize(st));
                 blob_bytes = t64[0] + t64[1];
                 GT_TRY(ctx->scratch_get(SC_ING_6, blob_bytes + 1, (void**)&d_blob));
-                ingest_key_names_kernel<<<igrid(ctx, kept), 256, 0, st>>>(kept, v_a, klen.u32(), (const unsigned long long*)soff.ptr,
+                ingest_key_names_kernel<<<grid_for(ctx, kept), 256, 0, st>>>(kept, v_a, klen.u32(), (const unsigned long long*)soff.ptr,
                                                                           (const char*)arena.ptr, d_noff, d_blob);
                 ctx->launches++;
             }
         }
-        ingest_key_ids_kernel<<<igrid(ctx, n), 256, 0, st>>>(n, k_a, kept, id.u32());
+        ingest_key_ids_kernel<<<grid_for(ctx, n), 256, 0, st>>>(n, k_a, kept, id.u32());
         ctx->launches++;
         GT_CUDA(cudaGetLastError());
     }
@@ -983,16 +999,16 @@ int32_t KeyTable::finish(gtgpu_ctx* ctx, uint32_t* n_kept, BufPtr* out_names, Bu
 // go into one KeyTable that keeps every barcode; after the last window the fragment tokenizer core runs once over the
 // accumulated fragments and their dense barcode ids.  With out_spans the barcodes come back as u32 (first byte, length) spans
 // into the text, else as names + u64 name offsets.  The caller holds ctx->mu.
-int32_t tokenize_fragments_file_locked(gtgpu_index* ix, const char* host_text, const char* dev_text, uint64_t n_bytes, uint32_t n_names,
-                                       const char* names, const uint32_t* name_offsets, uint32_t unk_id, const std::string& who,
-                                       uint32_t* out_n_barcodes, BufPtr* out_names, BufPtr* out_name_offsets, BufPtr* out_spans,
-                                       BufPtr* out_barcode_offsets, BufPtr* out_ids) {
+static int32_t tokenize_fragments_file_locked(gtgpu_index* ix, const Text& t, uint32_t n_names, const char* names,
+                                              const uint32_t* name_offsets, uint32_t unk_id, const std::string& who, uint32_t* out_n_barcodes,
+                                              BufPtr* out_names, BufPtr* out_name_offsets, BufPtr* out_spans, BufPtr* out_barcode_offsets,
+                                              BufPtr* out_ids) {
     gtgpu_ctx* ctx = ix->ctx;
     KeyTable tab(true, out_spans != nullptr, ~0ull, who, "gtgpu_tokenize_fragments", "barcode", "barcodes");
-    if (n_bytes) {
+    if (t.n_bytes) {
         NameTable nt;
         GT_TRY(upload_name_table(ctx, n_names, names, name_offsets, &nt));
-        GT_TRY(for_each_window(ctx, host_text, dev_text, n_bytes, who,
+        GT_TRY(for_each_window(ctx, t, who,
                                [&](const char* d, uint64_t nb, uint64_t byte0, uint64_t line0, uint32_t* n_lines) -> int32_t {
             ParsedLines fp;
             GT_TRY(parse_lines_locked(ctx, d, nb, FRAG_TOKENIZE, nt, BedFilesView{}, &fp));
@@ -1034,10 +1050,9 @@ __global__ void ingest_file_record_offsets_kernel(uint64_t n_files, const uint32
     }
 }
 
-int32_t parse_bed_files_locked(gtgpu_ctx* ctx, const char* host_text, const char* dev_text, uint64_t n_files, const uint64_t* file_offsets,
-                               const std::string& who, BedFilesRecords* out) {
+int32_t parse_bed_files_locked(gtgpu_ctx* ctx, const Text& t, const std::string& who, BedFilesRecords* out) {
     cudaStream_t st = ctx->stream;
-    const uint64_t n_bytes = file_offsets[n_files];
+    const uint64_t n_files = t.n_files, *file_offsets = t.file_offsets.data();
     DevMem d_fo, d_first_line, d_fs;
     GT_TRY(d_fo.reserve((n_files + 1) * 8, 0, st));
     GT_TRY(d_first_line.reserve(std::max<uint64_t>(n_files, 1) * 8, 0, st));
@@ -1045,8 +1060,7 @@ int32_t parse_bed_files_locked(gtgpu_ctx* ctx, const char* host_text, const char
     GT_CUDA(cudaStreamSynchronize(st));  // file_offsets is the caller's
     KeyTable tab(true, false, MAX_CHROM_NAMES, who, "gtgpu_igd_build", "chromosome", "chromosome names");
     std::vector<uint32_t> fs;  // the window's file starts that are not its first byte (window-relative)
-    GT_TRY(for_each_window(ctx, host_text, dev_text, n_bytes, who,
-                           [&](const char* d, uint64_t nb, uint64_t byte0, uint64_t line0, uint32_t* n_lines) -> int32_t {
+    GT_TRY(for_each_window(ctx, t, who, [&](const char* d, uint64_t nb, uint64_t byte0, uint64_t line0, uint32_t* n_lines) -> int32_t {
         fs.clear();
         for (const uint64_t* f = std::upper_bound(file_offsets, file_offsets + n_files + 1, byte0);
              f < file_offsets + n_files + 1 && *f < byte0 + nb; ++f)
@@ -1092,7 +1106,7 @@ int32_t parse_bed_files_locked(gtgpu_ctx* ctx, const char* host_text, const char
         DevMem roff;
         GT_TRY(roff.reserve((n_files + 1) * 8, 0, st));
         if (r.n) {
-            ingest_file_record_offsets_kernel<<<igrid(ctx, n_files + 1), 256, 0, st>>>(n_files, r.file.u32(), r.n,
+            ingest_file_record_offsets_kernel<<<grid_for(ctx, n_files + 1), 256, 0, st>>>(n_files, r.file.u32(), r.n,
                                                                                       (unsigned long long*)roff.ptr);
             ctx->launches++;
             GT_CUDA(cudaMemcpyAsync(r.file_offsets.data(), roff.ptr, (n_files + 1) * 8, cudaMemcpyDeviceToHost, st));
@@ -1126,10 +1140,9 @@ __global__ void ingest_remap_chr_kernel(uint64_t n, const uint32_t* __restrict__
     for (uint64_t i = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += stride) chr[i] = map[chr[i]];
 }
 
-int32_t parse_bed_queries_locked(gtgpu_ctx* ctx, const char* host_text, const char* dev_text, uint64_t n_files,
-                                 const uint64_t* file_offsets, uint32_t n_names, const char* names, const uint32_t* name_offsets,
+int32_t parse_bed_queries_locked(gtgpu_ctx* ctx, const Text& t, uint32_t n_names, const char* names, const uint32_t* name_offsets,
                                  bool with_rank, const std::string& who, BedFilesRecords* r, NameTable* nt) {
-    GT_TRY(parse_bed_files_locked(ctx, host_text, dev_text, n_files, file_offsets, who, r));
+    GT_TRY(parse_bed_files_locked(ctx, t, who, r));
     if (r->n == 0) return GTGPU_OK;
     cudaStream_t st = ctx->stream;
     GT_TRY(upload_name_table(ctx, n_names, names, name_offsets, nt, with_rank));  // scratch SC_SET_ID
@@ -1140,9 +1153,9 @@ int32_t parse_bed_queries_locked(gtgpu_ctx* ctx, const char* host_text, const ch
     GT_TRY(d_map.reserve((uint64_t)r->n_names * 4, 0, st));
     if (blob_bytes) GT_CUDA(cudaMemcpyAsync(d_blob.ptr, r->names->block.ptr, blob_bytes, cudaMemcpyHostToDevice, st));
     GT_CUDA(cudaMemcpyAsync(d_offs.ptr, r->name_offsets->block.ptr, ((uint64_t)r->n_names + 1) * 8, cudaMemcpyHostToDevice, st));
-    ingest_map_names_kernel<<<igrid(ctx, r->n_names), 256, 0, st>>>(r->n_names, (const char*)d_blob.ptr,
+    ingest_map_names_kernel<<<grid_for(ctx, r->n_names), 256, 0, st>>>(r->n_names, (const char*)d_blob.ptr,
                                                                      (const unsigned long long*)d_offs.ptr, *nt, d_map.u32());
-    ingest_remap_chr_kernel<<<igrid(ctx, r->n), 256, 0, st>>>(r->n, d_map.u32(), r->chr.u32());
+    ingest_remap_chr_kernel<<<grid_for(ctx, r->n), 256, 0, st>>>(r->n, d_map.u32(), r->chr.u32());
     ctx->launches += 2;
     GT_CUDA(cudaGetLastError());
     GT_CUDA(cudaStreamSynchronize(st));  // the map is freed here, and a later call may reuse the name table's scratch
@@ -1150,60 +1163,19 @@ int32_t parse_bed_queries_locked(gtgpu_ctx* ctx, const char* host_text, const ch
 }
 
 // ---- a batch of BED files tokenized in one pass: parse, per-file RegionSet::sort, fused find, [unk] rule ----------------------
-// The records arrive grouped by file in file order.  RegionSet::sort applies per file: stable by (chromosome string, start).  When
-// some file is out of order, stable radix passes by start, then chromosome rank, then file index (folded into the rank pass when
-// both fit 32 bits) give every file its own records in that order.  The caller holds ctx->mu.
-int32_t tokenize_bed_files_locked(gtgpu_index* ix, const char* host_text, const char* dev_text, uint64_t n_files,
-                                  const uint64_t* file_offsets, uint32_t n_names, const char* names, const uint32_t* name_offsets,
-                                  uint32_t unk_id, const std::string& who, uint64_t* out_file_token_offsets, BufPtr* out_ids) {
+// gtgpu_tokenize_bed_files on t.n_files > 0 files: out_file_token_offsets (n_files + 1, host) and *out_ids as gtgpu_tokenize_files
+// returns them.  The records arrive grouped by file in file order.  The caller holds ctx->mu.
+static int32_t tokenize_bed_files_locked(gtgpu_index* ix, const Text& t, uint32_t n_names, const char* names, const uint32_t* name_offsets,
+                                         uint32_t unk_id, const std::string& who, uint64_t* out_file_token_offsets, BufPtr* out_ids) {
     gtgpu_ctx* ctx = ix->ctx;
     cudaStream_t st = ctx->stream;
+    const uint64_t n_files = t.n_files;
     BedFilesRecords r;
     NameTable nt{};
-    GT_TRY(parse_bed_queries_locked(ctx, host_text, dev_text, n_files, file_offsets, n_names, names, name_offsets, true, who, &r, &nt));
+    GT_TRY(parse_bed_queries_locked(ctx, t, n_names, names, name_offsets, true, who, &r, &nt));
     const uint32_t n = (uint32_t)r.n;  // parse_bed_files_locked allows fewer than 2^32 - 1 records
     const uint32_t *q_chr = r.chr.u32(), *q_start = r.start.u32(), *q_end = r.end.u32();
-    uint32_t* d_flag;
-    GT_TRY(ctx->scratch_get(SC_MISC, 64, (void**)&d_flag));
-    GT_CUDA(cudaMemsetAsync(d_flag, 0, 4, st));
-    ingest_check_sorted_kernel<<<igrid(ctx, n), 256, 0, st>>>(n, q_chr, q_start, nt.rank, n_names, d_flag, r.file.u32());
-    ctx->launches++;
-    uint32_t unsorted = 0;
-    GT_CUDA(cudaMemcpyAsync(&unsorted, d_flag, 4, cudaMemcpyDeviceToHost, st));
-    GT_CUDA(cudaStreamSynchronize(st));
-    if (unsorted) {  // the parse's line scratch is free again; the find below does not touch it
-        uint32_t *k_a, *v_a, *k_b, *v_b;
-        GT_TRY(ctx->scratch_get(SC_ING_0, (size_t)n * 4, (void**)&k_a));
-        GT_TRY(ctx->scratch_get(SC_ING_1, (size_t)n * 4, (void**)&v_a));
-        GT_TRY(ctx->scratch_get(SC_ING_2, (size_t)n * 4, (void**)&k_b));
-        GT_TRY(ctx->scratch_get(SC_ING_3, (size_t)n * 4, (void**)&v_b));
-        void* d_tmp;
-        GT_TRY(ctx->scratch_get(SC_IN3_START, radix_sort_temp_bytes(n), &d_tmp));
-        GT_CUDA(cudaMemcpyAsync(k_a, q_start, (size_t)n * 4, cudaMemcpyDeviceToDevice, st));
-        ingest_iota_kernel<<<igrid(ctx, n), 256, 0, st>>>(n, v_a);
-        ctx->launches++;
-        int in_b = 0;
-        GT_TRY(radix_sort_pairs(ctx, n, k_a, v_a, k_b, v_b, 32, d_tmp, &in_b));
-        if (in_b) { std::swap(k_a, k_b); std::swap(v_a, v_b); }
-        int rank_bits = 1, file_bits = 1;
-        while (rank_bits < 32 && (1ull << rank_bits) < (uint64_t)n_names + 1) ++rank_bits;
-        while (file_bits < 32 && (1ull << file_bits) < n_files) ++file_bits;
-        const bool fold = rank_bits + file_bits <= 32;
-        ingest_rank_keys_kernel<<<igrid(ctx, n), 256, 0, st>>>(n, v_a, q_chr, nt.rank, n_names, k_a, fold ? r.file.u32() : nullptr,
-                                                              rank_bits);
-        ctx->launches++;
-        GT_TRY(radix_sort_pairs(ctx, n, k_a, v_a, k_b, v_b, fold ? rank_bits + file_bits : rank_bits, d_tmp, &in_b));
-        if (in_b) { std::swap(k_a, k_b); std::swap(v_a, v_b); }
-        if (!fold) {
-            GT_TRY(launch_gather_u32(ctx, n, r.file.u32(), v_a, k_a));
-            GT_TRY(radix_sort_pairs(ctx, n, k_a, v_a, k_b, v_b, file_bits, d_tmp, &in_b));
-            if (in_b) { std::swap(k_a, k_b); std::swap(v_a, v_b); }
-        }
-        // the order is v_a; the other three buffers take the sorted columns
-        ingest_gather_kernel<<<igrid(ctx, n), 256, 0, st>>>(n, v_a, q_chr, q_start, q_end, k_a, k_b, v_b);
-        ctx->launches++;
-        q_chr = k_a; q_start = k_b; q_end = v_b;
-    }
+    GT_TRY(sort_regions_locked(ctx, n, nt, n_names, r.file.u32(), n_files, &q_chr, &q_start, &q_end));
     // ---- fused find over the files, then the [unk] rule (Tokenizer::tokenize: a file without a token yields [unk]) ----------------
     uint64_t *d_fo, *d_raw_tok, *d_out_tok, total = 0;
     GT_TRY(ctx->scratch_get(SC_FILE_OFFS, (n_files + 1) * 8, (void**)&d_fo));
@@ -1229,6 +1201,137 @@ int32_t tokenize_bed_files_locked(gtgpu_index* ix, const char* host_text, const 
     return GTGPU_OK;
 }
 
+// the caller holds ctx->mu
+static int32_t tokenize_bed_locked(gtgpu_index* ix, const Text& t, uint32_t n_names, const char* names, const uint32_t* name_offsets,
+                                   uint32_t unk_id, gtgpu_buf** out_ids) {
+    gtgpu_ctx* ctx = ix->ctx;
+    const uint32_t *d_chr, *d_start, *d_end;
+    uint32_t* d_ids = nullptr;
+    uint64_t n = 0, total = 0;
+    GT_TRY(parse_bed_locked(ctx, t, n_names, names, name_offsets, &n, &d_chr, &d_start, &d_end));
+    GT_TRY(fused_find_all(ix, n, 0, nullptr, d_chr, d_start, d_end, nullptr, nullptr, &d_ids, &total));
+    BufPtr buf;
+    if (total == 0) {  // Tokenizer::tokenize: a call without a single token yields [unk] (tokenizer.rs:156-160)
+        GT_TRY(buf_new(ctx, 1, 4, &buf));
+        *reinterpret_cast<uint32_t*>(buf->block.ptr) = unk_id;
+        *out_ids = buf.release();
+        return GTGPU_OK;
+    }
+    const int32_t s = buf_from_device(ctx, d_ids, total, 4, ctx->stream, &buf);
+    if (s == GTGPU_ERR_CUDA) return fail(s, std::string("ingest: D2H: ") + gtgpu_last_error());
+    GT_TRY(s);
+    const cudaError_t e = cudaStreamSynchronize(ctx->stream);
+    if (e != cudaSuccess) return fail(GTGPU_ERR_CUDA, std::string("ingest: D2H: ") + cudaGetErrorString(e));
+    *out_ids = buf.release();
+    return GTGPU_OK;
+}
+
+// ---- the entry points: each plain-text / gzip pair shares one body ------------------------------------------------------------
+// A body checks its arguments, takes ctx->mu, opens the text (open_text_locked: gzip members are inflated whole into device
+// memory) and parses it where it is.  `who` is the entry point's name without "gtgpu_".
+
+static int32_t tokenize_bed_text(gtgpu_index* ix, const TextIn& in, const char* who, uint32_t n_names, const char* names,
+                                 const uint32_t* name_offsets, uint32_t unk_id, gtgpu_buf** out_ids) {
+    if (!ix || !out_ids || (n_names && (!names || !name_offsets))) return fail(GTGPU_ERR_INVALID, std::string(who) + ": null argument");
+    GT_TRY(in.check(who));
+    gtgpu_ctx* ctx = ix->ctx;
+    std::lock_guard<std::mutex> lk(ctx->mu);
+    GT_CUDA(cudaSetDevice(ctx->device));
+    Text t;
+    GT_TRY(open_text_locked(ctx, in, who, &t));
+    return tokenize_bed_locked(ix, t, n_names, names, name_offsets, unk_id, out_ids);
+}
+
+static int32_t tokenize_bed_files_text(gtgpu_index* ix, const TextIn& in, const char* who, uint32_t n_names, const char* names,
+                                       const uint32_t* name_offsets, uint32_t unk_id, uint64_t* out_file_token_offsets,
+                                       gtgpu_buf** out_ids) {
+    if (!ix || !out_file_token_offsets || !out_ids || (n_names && (!names || !name_offsets)))
+        return fail(GTGPU_ERR_INVALID, std::string(who) + ": null argument");
+    GT_TRY(in.check(who));
+    gtgpu_ctx* ctx = ix->ctx;
+    std::lock_guard<std::mutex> lk(ctx->mu);
+    GT_CUDA(cudaSetDevice(ctx->device));
+    BufPtr ids;
+    if (in.n_files == 0) {  // the offsets are [0] and the id buffer is empty
+        GT_TRY(buf_new(ctx, 0, 4, &ids));
+        out_file_token_offsets[0] = 0;
+    } else {
+        Text t;
+        GT_TRY(open_text_locked(ctx, in, who, &t));
+        GT_TRY(tokenize_bed_files_locked(ix, t, n_names, names, name_offsets, unk_id, who, out_file_token_offsets, &ids));
+    }
+    *out_ids = ids.release();
+    return GTGPU_OK;
+}
+
+// tokenize_fragment_file (fragments.rs:61-82) from the file's text, < 4 GiB: the barcodes come back as u32 spans into the text.
+// With out_text (gzip input) the inflated text comes back too, its copy on copy_out overlapping the parse.  The parse's errors
+// carry the text form's name.
+static int32_t tokenize_fragments_spans(gtgpu_index* ix, const TextIn& in, const char* who, uint32_t n_names, const char* names,
+                                        const uint32_t* name_offsets, uint32_t unk_id, uint32_t* out_n_barcodes,
+                                        gtgpu_buf** out_barcode_spans, gtgpu_buf** out_barcode_offsets, gtgpu_buf** out_ids,
+                                        gtgpu_buf** out_text) {
+    if (!ix || !out_n_barcodes || !out_barcode_spans || !out_barcode_offsets || !out_ids || (in.is_gz && !out_text) ||
+        (n_names && (!names || !name_offsets)))
+        return fail(GTGPU_ERR_INVALID, std::string(who) + ": null argument");
+    GT_TRY(in.check(who));
+    gtgpu_ctx* ctx = ix->ctx;
+    std::lock_guard<std::mutex> lk(ctx->mu);
+    GT_CUDA(cudaSetDevice(ctx->device));
+    Text t;
+    GT_TRY(open_text_locked(ctx, in, who, &t));
+    if (t.n_bytes >= 0xFFFFFFF0ull) return fail(GTGPU_ERR_UNSUPPORTED, "tokenize_fragments_text: at most 4 GiB of text per call");
+    BufPtr text, spans, offs, ids;
+    int32_t s = GTGPU_OK;
+    if (out_text) {
+        s = buf_from_device(ctx, t.bytes, t.n_bytes, 1, ctx->copy_out, &text);
+        if (s == GTGPU_ERR_CUDA) return fail(s, std::string(who) + ": D2H of the text failed");
+        GT_TRY(s);
+    }
+    try {
+        s = tokenize_fragments_file_locked(ix, t, n_names, names, name_offsets, unk_id, "tokenize_fragments_text", out_n_barcodes, nullptr,
+                                           nullptr, &spans, &offs, &ids);
+    } catch (...) {
+        cudaStreamSynchronize(ctx->copy_out);  // the text's copy ends before its block goes back to the cache
+        throw;
+    }
+    if (s == GTGPU_OK && out_text && cudaStreamSynchronize(ctx->copy_out) != cudaSuccess)
+        s = fail(GTGPU_ERR_CUDA, std::string(who) + ": D2H of the text failed");
+    if (s != GTGPU_OK) {
+        cudaStreamSynchronize(ctx->copy_out);
+        return s;
+    }
+    *out_barcode_spans = spans.release();
+    *out_barcode_offsets = offs.release();
+    *out_ids = ids.release();
+    if (out_text) *out_text = text.release();
+    return GTGPU_OK;
+}
+
+// tokenize_fragment_file from the file's text, any size: the barcodes come back as names.
+static int32_t tokenize_fragments_names(gtgpu_index* ix, const TextIn& in, const char* who, uint32_t n_names, const char* names,
+                                        const uint32_t* name_offsets, uint32_t unk_id, uint32_t* out_n_barcodes,
+                                        gtgpu_buf** out_barcode_names, gtgpu_buf** out_barcode_name_offsets,
+                                        gtgpu_buf** out_barcode_offsets, gtgpu_buf** out_ids) {
+    if (!ix || !out_n_barcodes || !out_barcode_names || !out_barcode_name_offsets || !out_barcode_offsets || !out_ids ||
+        (n_names && (!names || !name_offsets)))
+        return fail(GTGPU_ERR_INVALID, std::string(who) + ": null argument");
+    GT_TRY(in.check(who));
+    gtgpu_ctx* ctx = ix->ctx;
+    std::lock_guard<std::mutex> lk(ctx->mu);
+    GT_CUDA(cudaSetDevice(ctx->device));
+    Text t;
+    GT_TRY(open_text_locked(ctx, in, who, &t));
+    BufPtr nm, no, offs, ids;
+    GT_TRY(tokenize_fragments_file_locked(ix, t, n_names, names, name_offsets, unk_id, who, out_n_barcodes, &nm, &no, nullptr, &offs,
+                                          &ids));
+    *out_barcode_names = nm.release();
+    *out_barcode_name_offsets = no.release();
+    *out_barcode_offsets = offs.release();
+    *out_ids = ids.release();
+    return GTGPU_OK;
+}
+
 }  // namespace gtgpu
 
 using namespace gtgpu;
@@ -1240,9 +1343,11 @@ extern "C" int32_t gtgpu_parse_bed(gtgpu_ctx* ctx, const char* text, uint64_t n_
         return fail(GTGPU_ERR_INVALID, "parse_bed: null argument");
     std::lock_guard<std::mutex> lk(ctx->mu);
     GT_CUDA(cudaSetDevice(ctx->device));
-    uint32_t *d_chr, *d_start, *d_end;
+    Text t;
+    GT_TRY(open_text_locked(ctx, TextIn::plain(text, n_bytes), "parse_bed", &t));
+    const uint32_t *d_chr, *d_start, *d_end;
     uint64_t n = 0;
-    GT_TRY(parse_bed_locked(ctx, text, nullptr, n_bytes, n_names, names, name_offsets, &n, &d_chr, &d_start, &d_end));
+    GT_TRY(parse_bed_locked(ctx, t, n_names, names, name_offsets, &n, &d_chr, &d_start, &d_end));
     BufPtr bufs[3];
     const uint32_t* src[3] = {d_chr, d_start, d_end};
     for (int k = 0; k < 3; ++k) {
@@ -1261,135 +1366,65 @@ extern "C" int32_t gtgpu_parse_bed(gtgpu_ctx* ctx, const char* text, uint64_t n_
 
 extern "C" int32_t gtgpu_tokenize_bed(gtgpu_index* ix, const char* text, uint64_t n_bytes, uint32_t n_names, const char* names,
                                       const uint32_t* name_offsets, uint32_t unk_id, gtgpu_buf** out_ids) try {
-    if (!ix || !out_ids || (n_bytes && !text) || (n_names && (!names || !name_offsets)))
-        return fail(GTGPU_ERR_INVALID, "tokenize_bed: null argument");
-    gtgpu_ctx* ctx = ix->ctx;
-    std::lock_guard<std::mutex> lk(ctx->mu);
-    GT_CUDA(cudaSetDevice(ctx->device));
-    return tokenize_bed_locked(ix, text, nullptr, n_bytes, n_names, names, name_offsets, unk_id, out_ids);
+    return tokenize_bed_text(ix, TextIn::plain(text, n_bytes), "tokenize_bed", n_names, names, name_offsets, unk_id, out_ids);
 } GT_CATCH
 
-// the caller holds ctx->mu
-int32_t gtgpu::tokenize_bed_locked(gtgpu_index* ix, const char* host_text, const char* dev_text, uint64_t n_bytes, uint32_t n_names,
-                                   const char* names, const uint32_t* name_offsets, uint32_t unk_id, gtgpu_buf** out_ids) {
-    gtgpu_ctx* ctx = ix->ctx;
-    uint32_t *d_chr, *d_start, *d_end, *d_ids = nullptr;
-    uint64_t n = 0, total = 0;
-    GT_TRY(parse_bed_locked(ctx, host_text, dev_text, n_bytes, n_names, names, name_offsets, &n, &d_chr, &d_start, &d_end));
-    GT_TRY(fused_find_all(ix, n, 0, nullptr, d_chr, d_start, d_end, nullptr, nullptr, &d_ids, &total));
-    BufPtr buf;
-    if (total == 0) {  // Tokenizer::tokenize: a call without a single token yields [unk] (tokenizer.rs:156-160)
-        GT_TRY(buf_new(ctx, 1, 4, &buf));
-        *reinterpret_cast<uint32_t*>(buf->block.ptr) = unk_id;
-        *out_ids = buf.release();
-        return GTGPU_OK;
-    }
-    const int32_t s = buf_from_device(ctx, d_ids, total, 4, ctx->stream, &buf);
-    if (s == GTGPU_ERR_CUDA) return fail(s, std::string("ingest: D2H: ") + gtgpu_last_error());
-    GT_TRY(s);
-    const cudaError_t e = cudaStreamSynchronize(ctx->stream);
-    if (e != cudaSuccess) return fail(GTGPU_ERR_CUDA, std::string("ingest: D2H: ") + cudaGetErrorString(e));
-    *out_ids = buf.release();
-    return GTGPU_OK;
-}
-
-// n_files == 0: the offsets are [0] and the id buffer is empty
-static int32_t tokenize_no_files(gtgpu_ctx* ctx, uint64_t* out_file_token_offsets, gtgpu_buf** out_ids) {
-    BufPtr buf;
-    GT_TRY(buf_new(ctx, 0, 4, &buf));
-    out_file_token_offsets[0] = 0;
-    *out_ids = buf.release();
-    return GTGPU_OK;
-}
+// gtgpu_tokenize_bed on gzip members: inflate on the device, parse + sort + tokenize the text where it is.
+extern "C" int32_t gtgpu_tokenize_bed_gz(gtgpu_index* ix, uint64_t n_members, const uint8_t* gz, const uint64_t* member_offsets,
+                                         uint32_t n_names, const char* names, const uint32_t* name_offsets, uint32_t unk_id,
+                                         gtgpu_buf** out_ids) try {
+    return tokenize_bed_text(ix, TextIn::gzip(n_members, gz, member_offsets), "tokenize_bed_gz", n_names, names, name_offsets, unk_id,
+                             out_ids);
+} GT_CATCH
 
 extern "C" int32_t gtgpu_tokenize_bed_files(gtgpu_index* ix, uint64_t n_files, const char* text, const uint64_t* file_offsets,
                                             uint32_t n_names, const char* names, const uint32_t* name_offsets, uint32_t unk_id,
                                             uint64_t* out_file_token_offsets, gtgpu_buf** out_ids) try {
-    if (!ix || !file_offsets || !out_file_token_offsets || !out_ids || (n_names && (!names || !name_offsets)))
-        return fail(GTGPU_ERR_INVALID, "tokenize_bed_files: null argument");
-    if (file_offsets[0] != 0) return fail(GTGPU_ERR_INVALID, "tokenize_bed_files: file_offsets[0] must be 0");
-    for (uint64_t f = 0; f < n_files; ++f)
-        if (file_offsets[f] > file_offsets[f + 1]) return fail(GTGPU_ERR_INVALID, "tokenize_bed_files: file_offsets not monotone");
-    if (file_offsets[n_files] && !text) return fail(GTGPU_ERR_INVALID, "tokenize_bed_files: null text");
-    if (n_files >= 0xFFFFFFFFull) return fail(GTGPU_ERR_UNSUPPORTED, "tokenize_bed_files: too many files");
-    gtgpu_ctx* ctx = ix->ctx;
-    std::lock_guard<std::mutex> lk(ctx->mu);
-    GT_CUDA(cudaSetDevice(ctx->device));
-    if (n_files == 0) return tokenize_no_files(ctx, out_file_token_offsets, out_ids);
-    BufPtr ids;
-    GT_TRY(tokenize_bed_files_locked(ix, text, nullptr, n_files, file_offsets, n_names, names, name_offsets, unk_id, "tokenize_bed_files",
-                                     out_file_token_offsets, &ids));
-    *out_ids = ids.release();
-    return GTGPU_OK;
+    return tokenize_bed_files_text(ix, TextIn::plain(text, n_files, file_offsets), "tokenize_bed_files", n_names, names, name_offsets,
+                                   unk_id, out_file_token_offsets, out_ids);
 } GT_CATCH
 
 extern "C" int32_t gtgpu_tokenize_bed_files_gz(gtgpu_index* ix, uint64_t n_files, const uint64_t* file_members, uint64_t n_members,
                                                const uint8_t* gz, const uint64_t* member_offsets, uint32_t n_names, const char* names,
                                                const uint32_t* name_offsets, uint32_t unk_id, uint64_t* out_file_token_offsets,
                                                gtgpu_buf** out_ids) try {
-    if (!ix || !file_members || !out_file_token_offsets || !out_ids || (n_names && (!names || !name_offsets)))
-        return fail(GTGPU_ERR_INVALID, "tokenize_bed_files_gz: null argument");
-    GT_TRY(check_members(n_members, gz, member_offsets, "tokenize_bed_files_gz"));
-    if (file_members[0] != 0 || file_members[n_files] != n_members)
-        return fail(GTGPU_ERR_INVALID, "tokenize_bed_files_gz: file_members must run from 0 to n_members");
-    for (uint64_t f = 0; f < n_files; ++f)
-        if (file_members[f] > file_members[f + 1]) return fail(GTGPU_ERR_INVALID, "tokenize_bed_files_gz: file_members not monotone");
-    if (n_files >= 0xFFFFFFFFull) return fail(GTGPU_ERR_UNSUPPORTED, "tokenize_bed_files_gz: too many files");
-    gtgpu_ctx* ctx = ix->ctx;
-    std::lock_guard<std::mutex> lk(ctx->mu);
-    GT_CUDA(cudaSetDevice(ctx->device));
-    if (n_files == 0) return tokenize_no_files(ctx, out_file_token_offsets, out_ids);
-    uint8_t* d_text = nullptr;
-    uint64_t n_text = 0;
-    std::vector<uint64_t> text_offsets(n_members + 1), fo(n_files + 1);
-    GT_TRY(inflate_whole_locked(ctx, n_members, gz, member_offsets, "tokenize_bed_files_gz", &d_text, &n_text, text_offsets.data()));
-    for (uint64_t f = 0; f <= n_files; ++f) fo[f] = text_offsets[file_members[f]];
-    BufPtr ids;
-    GT_TRY(tokenize_bed_files_locked(ix, nullptr, (const char*)d_text, n_files, fo.data(), n_names, names, name_offsets, unk_id,
-                                     "tokenize_bed_files_gz", out_file_token_offsets, &ids));
-    *out_ids = ids.release();
-    return GTGPU_OK;
+    return tokenize_bed_files_text(ix, TextIn::gzip(n_members, gz, member_offsets, n_files, file_members), "tokenize_bed_files_gz",
+                                   n_names, names, name_offsets, unk_id, out_file_token_offsets, out_ids);
 } GT_CATCH
 
-// tokenize_fragment_file (fragments.rs:61-82) from the file's text, < 4 GiB: the barcodes come back as u32 spans into the text.
 extern "C" int32_t gtgpu_tokenize_fragments_text(gtgpu_index* ix, const char* text, uint64_t n_bytes, uint32_t n_names,
                                                  const char* names, const uint32_t* name_offsets, uint32_t unk_id,
                                                  uint32_t* out_n_barcodes, gtgpu_buf** out_barcode_spans,
                                                  gtgpu_buf** out_barcode_offsets, gtgpu_buf** out_ids) try {
-    if (!ix || !out_n_barcodes || !out_barcode_spans || !out_barcode_offsets || !out_ids || (n_bytes && !text) ||
-        (n_names && (!names || !name_offsets)))
-        return fail(GTGPU_ERR_INVALID, "tokenize_fragments_text: null argument");
-    if (n_bytes >= 0xFFFFFFF0ull) return fail(GTGPU_ERR_UNSUPPORTED, "tokenize_fragments_text: at most 4 GiB of text per call");
-    gtgpu_ctx* ctx = ix->ctx;
-    std::lock_guard<std::mutex> lk(ctx->mu);
-    GT_CUDA(cudaSetDevice(ctx->device));
-    BufPtr spans, offs, ids;
-    GT_TRY(tokenize_fragments_file_locked(ix, text, nullptr, n_bytes, n_names, names, name_offsets, unk_id, "tokenize_fragments_text",
-                                          out_n_barcodes, nullptr, nullptr, &spans, &offs, &ids));
-    *out_barcode_spans = spans.release();
-    *out_barcode_offsets = offs.release();
-    *out_ids = ids.release();
-    return GTGPU_OK;
+    return tokenize_fragments_spans(ix, TextIn::plain(text, n_bytes), "tokenize_fragments_text", n_names, names, name_offsets, unk_id,
+                                    out_n_barcodes, out_barcode_spans, out_barcode_offsets, out_ids, nullptr);
 } GT_CATCH
 
-// tokenize_fragment_file from the file's text, any size: the barcodes come back as names.
+// gtgpu_tokenize_fragments_text on gzip members (a bgzip'ed fragment file: thousands of members).  *out_text returns the
+// inflated text as well: the barcode spans index into it.
+extern "C" int32_t gtgpu_tokenize_fragments_gz(gtgpu_index* ix, uint64_t n_members, const uint8_t* gz, const uint64_t* member_offsets,
+                                               uint32_t n_names, const char* names, const uint32_t* name_offsets, uint32_t unk_id,
+                                               uint32_t* out_n_barcodes, gtgpu_buf** out_barcode_spans,
+                                               gtgpu_buf** out_barcode_offsets, gtgpu_buf** out_ids, gtgpu_buf** out_text) try {
+    return tokenize_fragments_spans(ix, TextIn::gzip(n_members, gz, member_offsets), "tokenize_fragments_gz", n_names, names,
+                                    name_offsets, unk_id, out_n_barcodes, out_barcode_spans, out_barcode_offsets, out_ids, out_text);
+} GT_CATCH
+
 extern "C" int32_t gtgpu_tokenize_fragments_file(gtgpu_index* ix, const char* text, uint64_t n_bytes, uint32_t n_names,
                                                  const char* names, const uint32_t* name_offsets, uint32_t unk_id,
                                                  uint32_t* out_n_barcodes, gtgpu_buf** out_barcode_names,
                                                  gtgpu_buf** out_barcode_name_offsets, gtgpu_buf** out_barcode_offsets,
                                                  gtgpu_buf** out_ids) try {
-    if (!ix || !out_n_barcodes || !out_barcode_names || !out_barcode_name_offsets || !out_barcode_offsets || !out_ids ||
-        (n_bytes && !text) || (n_names && (!names || !name_offsets)))
-        return fail(GTGPU_ERR_INVALID, "tokenize_fragments_file: null argument");
-    gtgpu_ctx* ctx = ix->ctx;
-    std::lock_guard<std::mutex> lk(ctx->mu);
-    GT_CUDA(cudaSetDevice(ctx->device));
-    BufPtr nm, no, offs, ids;
-    GT_TRY(tokenize_fragments_file_locked(ix, text, nullptr, n_bytes, n_names, names, name_offsets, unk_id, "tokenize_fragments_file",
-                                          out_n_barcodes, &nm, &no, nullptr, &offs, &ids));
-    *out_barcode_names = nm.release();
-    *out_barcode_name_offsets = no.release();
-    *out_barcode_offsets = offs.release();
-    *out_ids = ids.release();
-    return GTGPU_OK;
+    return tokenize_fragments_names(ix, TextIn::plain(text, n_bytes), "tokenize_fragments_file", n_names, names, name_offsets, unk_id,
+                                    out_n_barcodes, out_barcode_names, out_barcode_name_offsets, out_barcode_offsets, out_ids);
+} GT_CATCH
+
+extern "C" int32_t gtgpu_tokenize_fragments_file_gz(gtgpu_index* ix, uint64_t n_members, const uint8_t* gz, const uint64_t* member_offsets,
+                                                    uint32_t n_names, const char* names, const uint32_t* name_offsets, uint32_t unk_id,
+                                                    uint32_t* out_n_barcodes, gtgpu_buf** out_barcode_names,
+                                                    gtgpu_buf** out_barcode_name_offsets, gtgpu_buf** out_barcode_offsets,
+                                                    gtgpu_buf** out_ids) try {
+    return tokenize_fragments_names(ix, TextIn::gzip(n_members, gz, member_offsets), "tokenize_fragments_file_gz", n_names, names,
+                                    name_offsets, unk_id, out_n_barcodes, out_barcode_names, out_barcode_name_offsets,
+                                    out_barcode_offsets, out_ids);
 } GT_CATCH

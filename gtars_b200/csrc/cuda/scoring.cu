@@ -99,16 +99,6 @@ __global__ void score_barcode_offsets_kernel(uint32_t n_barcodes, uint64_t nnz, 
     out[b] = lo;
 }
 
-static int grid_for(gtgpu_ctx* ctx, uint64_t n) {
-    return (int)std::max<uint64_t>(1, std::min<uint64_t>((n + 255) / 256, (uint64_t)ctx->sm_count * 16));
-}
-
-static int bits_for(uint64_t n_values) {
-    int bits = 1;
-    while (bits < 32 && (1ull << bits) < n_values) ++bits;
-    return bits;
-}
-
 // Shared front end: fused find over device-resident queries with the optimistic capacity + exact re-run protocol.
 // Returns the raw ids in SC_OUT_IDS (*d_ids) and their number.
 int32_t fused_find_all(gtgpu_index* ix, uint64_t nq, uint64_t n_files, const uint64_t* d_qfo, const uint32_t* d_qc,
@@ -288,10 +278,10 @@ static int32_t score_barcodes_dev_locked(gtgpu_index* ix, uint64_t n, const uint
             // stable LSD: by peak first, then by barcode -> sorted by (barcode, peak)
             uint32_t *ka = d_ids, *va = d_hbc, *kb = d_k2, *vb = d_v2;
             int in_b = 0;
-            GT_TRY(radix_sort_pairs(ctx, total, ka, va, kb, vb, bits_for((uint64_t)ix->max_val + 1), d_tmp, &in_b));
+            GT_TRY(radix_sort_pairs(ctx, total, ka, va, kb, vb, bits_for_value(ix->max_val), d_tmp, &in_b));
             if (in_b) { std::swap(ka, kb); std::swap(va, vb); }
             // now (ka = peaks sorted, va = barcodes); second sort keys = barcodes, values = peaks
-            GT_TRY(radix_sort_pairs(ctx, total, va, ka, vb, kb, bits_for(n_barcodes), d_tmp, &in_b));
+            GT_TRY(radix_sort_pairs(ctx, total, va, ka, vb, kb, bits_for_value(n_barcodes ? n_barcodes - 1 : 0), d_tmp, &in_b));
             uint32_t* s_bc = in_b ? vb : va;
             uint32_t* s_pk = in_b ? kb : ka;
             GT_TRY(ctx->scratch_get(SC_COUNTS, total * 8, (void**)&d_head));
@@ -362,7 +352,8 @@ extern "C" int32_t gtgpu_score_barcodes(gtgpu_index* ix, uint64_t n, const uint3
 } GT_CATCH
 
 // ---- region / barcode scoring from a fragment file's bytes -----------------------------------------------------------------
-// Each file is parsed in windows (for_each_window, ingest.cu); gzip members are inflated whole into device memory first.
+// Each file is parsed in windows (for_each_window, ingest.cu); gzip members are inflated whole into device memory first
+// (open_text_locked).
 namespace gtgpu {
 
 static int32_t parse_error(const std::string& who, uint64_t line) {
@@ -374,22 +365,20 @@ static int32_t too_many(const std::string& who) {
 }
 
 // the caller holds ctx->mu
-static int32_t score_matrix_text_locked(gtgpu_index* ix, const char* host_text, const char* dev_text, uint64_t n_bytes,
-                                        uint32_t n_names, const char* names, const uint32_t* name_offsets, int32_t mode,
-                                        uint64_t n_cols, uint32_t* out_row, const std::string& who) {
+static int32_t score_matrix_text_locked(gtgpu_index* ix, const Text& t, uint32_t n_names, const char* names, const uint32_t* name_offsets,
+                                        int32_t mode, uint64_t n_cols, uint32_t* out_row, const std::string& who) {
     gtgpu_ctx* ctx = ix->ctx;
     cudaStream_t st = ctx->stream;
     uint32_t* d_row;
     GT_TRY(ctx->scratch_get(SC_MATRIX, std::max<uint64_t>(n_cols * 4, 4), (void**)&d_row));
     GT_CUDA(cudaMemsetAsync(d_row, 0, n_cols * 4, st));
-    if (n_bytes) {
+    if (t.n_bytes) {
         NameTable nt;
         uint64_t* d_fo;
         uint64_t total = 0;
         GT_TRY(upload_name_table(ctx, n_names, names, name_offsets, &nt));
         GT_TRY(ctx->scratch_get(SC_FILE_OFFS, 16, (void**)&d_fo));
-        GT_TRY(for_each_window(ctx, host_text, dev_text, n_bytes, who,
-                               [&](const char* d, uint64_t nb, uint64_t, uint64_t line0, uint32_t* n_lines) -> int32_t {
+        GT_TRY(for_each_window(ctx, t, who, [&](const char* d, uint64_t nb, uint64_t, uint64_t line0, uint32_t* n_lines) -> int32_t {
             ParsedLines fp;
             GT_TRY(parse_lines_locked(ctx, d, nb, FRAG_SCORE_MATRIX, nt, BedFilesView{}, &fp));
             *n_lines = fp.n_lines;
@@ -409,17 +398,16 @@ static int32_t score_matrix_text_locked(gtgpu_index* ix, const char* host_text, 
 }
 
 // the caller holds ctx->mu
-static int32_t score_barcodes_text_locked(gtgpu_index* ix, const char* host_text, const char* dev_text, uint64_t n_bytes,
-                                          uint32_t n_names, const char* names, const uint32_t* name_offsets, uint32_t* out_n_barcodes,
+static int32_t score_barcodes_text_locked(gtgpu_index* ix, const Text& t, uint32_t n_names, const char* names,
+                                          const uint32_t* name_offsets, uint32_t* out_n_barcodes,
                                           gtgpu_buf** out_names, gtgpu_buf** out_name_offsets, gtgpu_buf** out_barcode_offsets,
                                           gtgpu_buf** out_peaks, gtgpu_buf** out_counts, const std::string& who) {
     gtgpu_ctx* ctx = ix->ctx;
     KeyTable tab(false, false, ~0ull, who, "gtgpu_score_barcodes", "barcode", "barcodes");
-    if (n_bytes) {
+    if (t.n_bytes) {
         NameTable nt;
         GT_TRY(upload_name_table(ctx, n_names, names, name_offsets, &nt));
-        GT_TRY(for_each_window(ctx, host_text, dev_text, n_bytes, who,
-                               [&](const char* d, uint64_t nb, uint64_t byte0, uint64_t line0, uint32_t* n_lines) -> int32_t {
+        GT_TRY(for_each_window(ctx, t, who, [&](const char* d, uint64_t nb, uint64_t byte0, uint64_t line0, uint32_t* n_lines) -> int32_t {
             ParsedLines fp;
             GT_TRY(parse_lines_locked(ctx, d, nb, FRAG_SCORE_BARCODES, nt, BedFilesView{}, &fp));
             *n_lines = fp.n_lines;
@@ -441,64 +429,63 @@ static int32_t score_barcodes_text_locked(gtgpu_index* ix, const char* host_text
     return GTGPU_OK;
 }
 
+// The bodies of the plain-text / gzip entry point pairs (`who`: the entry point's name without "gtgpu_")
+static int32_t score_matrix_text(gtgpu_index* ix, const TextIn& in, const char* who, uint32_t n_names, const char* names,
+                                 const uint32_t* name_offsets, int32_t mode, uint64_t n_cols, uint32_t* out_row) {
+    if (!ix || (n_cols && !out_row) || (n_names && (!names || !name_offsets))) return fail(GTGPU_ERR_INVALID, std::string(who) + ": null argument");
+    if (mode != GTGPU_SCORE_ATAC && mode != GTGPU_SCORE_CHIP) return fail(GTGPU_ERR_INVALID, std::string(who) + ": unknown mode");
+    GT_TRY(in.check(who));
+    gtgpu_ctx* ctx = ix->ctx;
+    std::lock_guard<std::mutex> lk(ctx->mu);
+    GT_CUDA(cudaSetDevice(ctx->device));
+    Text t;
+    GT_TRY(open_text_locked(ctx, in, who, &t));
+    return score_matrix_text_locked(ix, t, n_names, names, name_offsets, mode, n_cols, out_row, who);
+}
+
+static int32_t score_barcodes_text(gtgpu_index* ix, const TextIn& in, const char* who, uint32_t n_names, const char* names,
+                                   const uint32_t* name_offsets, uint32_t* out_n_barcodes, gtgpu_buf** out_barcode_names,
+                                   gtgpu_buf** out_barcode_name_offsets, gtgpu_buf** out_barcode_offsets, gtgpu_buf** out_peaks,
+                                   gtgpu_buf** out_counts) {
+    if (!ix || !out_n_barcodes || !out_barcode_names || !out_barcode_name_offsets || !out_barcode_offsets || !out_peaks || !out_counts ||
+        (n_names && (!names || !name_offsets)))
+        return fail(GTGPU_ERR_INVALID, std::string(who) + ": null argument");
+    GT_TRY(in.check(who));
+    gtgpu_ctx* ctx = ix->ctx;
+    std::lock_guard<std::mutex> lk(ctx->mu);
+    GT_CUDA(cudaSetDevice(ctx->device));
+    Text t;
+    GT_TRY(open_text_locked(ctx, in, who, &t));
+    return score_barcodes_text_locked(ix, t, n_names, names, name_offsets, out_n_barcodes, out_barcode_names, out_barcode_name_offsets,
+                                      out_barcode_offsets, out_peaks, out_counts, who);
+}
+
 }  // namespace gtgpu
 
 extern "C" int32_t gtgpu_score_matrix_text(gtgpu_index* ix, const char* text, uint64_t n_bytes, uint32_t n_names, const char* names,
                                            const uint32_t* name_offsets, int32_t mode, uint64_t n_cols, uint32_t* out_row) try {
-    if (!ix || (n_cols && !out_row) || (n_bytes && !text) || (n_names && (!names || !name_offsets)))
-        return fail(GTGPU_ERR_INVALID, "score_matrix_text: null argument");
-    if (mode != GTGPU_SCORE_ATAC && mode != GTGPU_SCORE_CHIP) return fail(GTGPU_ERR_INVALID, "score_matrix_text: unknown mode");
-    gtgpu_ctx* ctx = ix->ctx;
-    std::lock_guard<std::mutex> lk(ctx->mu);
-    GT_CUDA(cudaSetDevice(ctx->device));
-    return score_matrix_text_locked(ix, text, nullptr, n_bytes, n_names, names, name_offsets, mode, n_cols, out_row, "score_matrix_text");
+    return score_matrix_text(ix, TextIn::plain(text, n_bytes), "score_matrix_text", n_names, names, name_offsets, mode, n_cols, out_row);
 } GT_CATCH
 
 extern "C" int32_t gtgpu_score_matrix_gz(gtgpu_index* ix, uint64_t n_members, const uint8_t* gz, const uint64_t* member_offsets,
                                          uint32_t n_names, const char* names, const uint32_t* name_offsets, int32_t mode, uint64_t n_cols,
                                          uint32_t* out_row) try {
-    if (!ix || (n_cols && !out_row) || (n_names && (!names || !name_offsets))) return fail(GTGPU_ERR_INVALID, "score_matrix_gz: null argument");
-    if (mode != GTGPU_SCORE_ATAC && mode != GTGPU_SCORE_CHIP) return fail(GTGPU_ERR_INVALID, "score_matrix_gz: unknown mode");
-    GT_TRY(check_members(n_members, gz, member_offsets, "score_matrix_gz"));
-    gtgpu_ctx* ctx = ix->ctx;
-    std::lock_guard<std::mutex> lk(ctx->mu);
-    GT_CUDA(cudaSetDevice(ctx->device));
-    uint8_t* d_text = nullptr;
-    uint64_t n_text = 0;
-    GT_TRY(inflate_whole_locked(ctx, n_members, gz, member_offsets, "score_matrix_gz", &d_text, &n_text));
-    return score_matrix_text_locked(ix, nullptr, (const char*)d_text, n_text, n_names, names, name_offsets, mode, n_cols, out_row,
-                                    "score_matrix_gz");
+    return score_matrix_text(ix, TextIn::gzip(n_members, gz, member_offsets), "score_matrix_gz", n_names, names, name_offsets, mode,
+                             n_cols, out_row);
 } GT_CATCH
 
 extern "C" int32_t gtgpu_score_barcodes_text(gtgpu_index* ix, const char* text, uint64_t n_bytes, uint32_t n_names, const char* names,
                                              const uint32_t* name_offsets, uint32_t* out_n_barcodes, gtgpu_buf** out_barcode_names,
                                              gtgpu_buf** out_barcode_name_offsets, gtgpu_buf** out_barcode_offsets,
                                              gtgpu_buf** out_peaks, gtgpu_buf** out_counts) try {
-    if (!ix || !out_n_barcodes || !out_barcode_names || !out_barcode_name_offsets || !out_barcode_offsets || !out_peaks || !out_counts ||
-        (n_bytes && !text) || (n_names && (!names || !name_offsets)))
-        return fail(GTGPU_ERR_INVALID, "score_barcodes_text: null argument");
-    gtgpu_ctx* ctx = ix->ctx;
-    std::lock_guard<std::mutex> lk(ctx->mu);
-    GT_CUDA(cudaSetDevice(ctx->device));
-    return score_barcodes_text_locked(ix, text, nullptr, n_bytes, n_names, names, name_offsets, out_n_barcodes, out_barcode_names,
-                                      out_barcode_name_offsets, out_barcode_offsets, out_peaks, out_counts, "score_barcodes_text");
+    return score_barcodes_text(ix, TextIn::plain(text, n_bytes), "score_barcodes_text", n_names, names, name_offsets, out_n_barcodes,
+                               out_barcode_names, out_barcode_name_offsets, out_barcode_offsets, out_peaks, out_counts);
 } GT_CATCH
 
 extern "C" int32_t gtgpu_score_barcodes_gz(gtgpu_index* ix, uint64_t n_members, const uint8_t* gz, const uint64_t* member_offsets,
                                            uint32_t n_names, const char* names, const uint32_t* name_offsets, uint32_t* out_n_barcodes,
                                            gtgpu_buf** out_barcode_names, gtgpu_buf** out_barcode_name_offsets,
                                            gtgpu_buf** out_barcode_offsets, gtgpu_buf** out_peaks, gtgpu_buf** out_counts) try {
-    if (!ix || !out_n_barcodes || !out_barcode_names || !out_barcode_name_offsets || !out_barcode_offsets || !out_peaks || !out_counts ||
-        (n_names && (!names || !name_offsets)))
-        return fail(GTGPU_ERR_INVALID, "score_barcodes_gz: null argument");
-    GT_TRY(check_members(n_members, gz, member_offsets, "score_barcodes_gz"));
-    gtgpu_ctx* ctx = ix->ctx;
-    std::lock_guard<std::mutex> lk(ctx->mu);
-    GT_CUDA(cudaSetDevice(ctx->device));
-    uint8_t* d_text = nullptr;
-    uint64_t n_text = 0;
-    GT_TRY(inflate_whole_locked(ctx, n_members, gz, member_offsets, "score_barcodes_gz", &d_text, &n_text));
-    return score_barcodes_text_locked(ix, nullptr, (const char*)d_text, n_text, n_names, names, name_offsets, out_n_barcodes,
-                                      out_barcode_names, out_barcode_name_offsets, out_barcode_offsets, out_peaks, out_counts,
-                                      "score_barcodes_gz");
+    return score_barcodes_text(ix, TextIn::gzip(n_members, gz, member_offsets), "score_barcodes_gz", n_names, names, name_offsets,
+                               out_n_barcodes, out_barcode_names, out_barcode_name_offsets, out_barcode_offsets, out_peaks, out_counts);
 } GT_CATCH

@@ -631,18 +631,32 @@ static void read_raw_bytes(const std::string& path, std::string& raw) {
     if (size > 0 && !f.read(&raw[0], size)) throw Error("Failed to read file: \"" + path + "\"");
 }
 
-static bool gz_members_for_device(const std::string& path, std::string& raw, std::vector<uint64_t>& members) {
-    if (!ends_with_gz(path)) return false;
-    read_raw_bytes(path, raw);
+// the n_members + 1 offsets of the gzip members of raw (gtgpu_gzip_members: BGZF blocks split, else one member)
+static std::vector<uint64_t> gzip_member_offsets(const std::string& raw) {
     uint64_t n = 0;
     gtgpu_gzip_members((const uint8_t*)raw.data(), raw.size(), 0, nullptr, &n);  // count only
-    if (n < 16) return false;
-    members.resize(n + 1);
-    check(gtgpu_gzip_members((const uint8_t*)raw.data(), raw.size(), members.size(), members.data(), &n), "gtgpu_gzip_members");
-    return true;
+    std::vector<uint64_t> m(n + 1, 0);
+    check(gtgpu_gzip_members((const uint8_t*)raw.data(), raw.size(), m.size(), m.data(), &n), "gtgpu_gzip_members");
+    return m;
 }
 
 namespace {
+// One file's bytes for a device parser: a .gz file of at least 16 members (bgzip'ed) stays gzip for the device inflater, any other
+// file is read by read_file_bytes (a single-member gzip is inflated by zlib on the host).
+struct FileBytes {
+    std::string raw, text;
+    std::vector<uint64_t> members;
+    bool gz = false;
+    explicit FileBytes(const std::string& path) {
+        if (ends_with_gz(path)) {
+            read_raw_bytes(path, raw);
+            members = gzip_member_offsets(raw);
+            gz = members.size() - 1 >= 16;
+        }
+        if (!gz) text = read_file_bytes(path);
+    }
+};
+
 // The bytes of n BED files for one device call.  When every path ends in ".gz" they stay gzip: every file's bytes back to back
 // with their member offsets, for the device inflater.  Otherwise the texts go back to back (".gz" inflated by zlib).
 struct BedFilesBytes {
@@ -659,14 +673,10 @@ BedFilesBytes gather_bed_files(const std::vector<std::string>& paths) {
         // one-member .bed.gz files are the common case: every member of every file is inflated on the device in parallel
         b.gz = true;
         std::string raw;
-        std::vector<uint64_t> m;
         for (const auto& p : paths) {
             read_raw_bytes(p, raw);
-            uint64_t n = 0;
-            gtgpu_gzip_members((const uint8_t*)raw.data(), raw.size(), 0, nullptr, &n);  // count only
-            m.assign(n + 1, 0);
-            check(gtgpu_gzip_members((const uint8_t*)raw.data(), raw.size(), m.size(), m.data(), &n), "gtgpu_gzip_members");
-            for (uint64_t k = 1; k <= n; ++k) b.members.push_back(b.raw.size() + m[k]);
+            const std::vector<uint64_t> m = gzip_member_offsets(raw);
+            for (uint64_t k = 1; k < m.size(); ++k) b.members.push_back(b.raw.size() + m[k]);
             b.file_members.push_back(b.members.size() - 1);
             b.raw += raw;
         }
@@ -719,18 +729,15 @@ BedFilesBytes gather_bed_files(const std::vector<std::string>& paths) {
 std::vector<uint32_t> Tokenizer::encode_bed_file(const std::string& path) const {
     NameBlob nb(cmap_);
     PinnedResult ids;
-    std::string raw;
-    std::vector<uint64_t> members;
-    if (gz_members_for_device(path, raw, members)) {
-        check(gtgpu_tokenize_bed_gz(index_, members.size() - 1, (const uint8_t*)raw.data(), members.data(), (uint32_t)cmap_.size(),
+    const FileBytes fb(path);
+    if (fb.gz)
+        check(gtgpu_tokenize_bed_gz(index_, fb.members.size() - 1, (const uint8_t*)fb.raw.data(), fb.members.data(), (uint32_t)cmap_.size(),
                                     nb.blob.data(), nb.offsets.data(), unk_id_, &ids.buf),
               "gtgpu_tokenize_bed_gz");
-        return std::vector<uint32_t>(ids.data(), ids.data() + ids.len());
-    }
-    const std::string text = read_file_bytes(path);
-    check(gtgpu_tokenize_bed(index_, text.data(), text.size(), (uint32_t)cmap_.size(), nb.blob.data(), nb.offsets.data(), unk_id_,
-                             &ids.buf),
-          "gtgpu_tokenize_bed");
+    else
+        check(gtgpu_tokenize_bed(index_, fb.text.data(), fb.text.size(), (uint32_t)cmap_.size(), nb.blob.data(), nb.offsets.data(), unk_id_,
+                                 &ids.buf),
+              "gtgpu_tokenize_bed");
     return std::vector<uint32_t>(ids.data(), ids.data() + ids.len());
 }
 
@@ -821,20 +828,17 @@ std::vector<std::pair<std::string, std::vector<uint32_t>>> Tokenizer::tokenize_f
     uint32_t n_barcodes = 0;
     PinnedResult names, name_offsets, offs, ids;
     {
-        std::string raw;
-        std::vector<uint64_t> members;
-        if (gz_members_for_device(path, raw, members)) {  // bgzip'ed fragment file: inflated and parsed on the device
-            check(gtgpu_tokenize_fragments_file_gz(index_, members.size() - 1, (const uint8_t*)raw.data(), members.data(),
+        const FileBytes fb(path);
+        if (fb.gz)  // bgzip'ed fragment file: inflated and parsed on the device
+            check(gtgpu_tokenize_fragments_file_gz(index_, fb.members.size() - 1, (const uint8_t*)fb.raw.data(), fb.members.data(),
                                                    (uint32_t)cmap_.size(), nb.blob.data(), nb.offsets.data(), unk_id_, &n_barcodes,
                                                    &names.buf, &name_offsets.buf, &offs.buf, &ids.buf),
                   "gtgpu_tokenize_fragments_file_gz");
-        } else {
-            const std::string text = read_file_bytes(path);
-            check(gtgpu_tokenize_fragments_file(index_, text.data(), text.size(), (uint32_t)cmap_.size(), nb.blob.data(),
+        else
+            check(gtgpu_tokenize_fragments_file(index_, fb.text.data(), fb.text.size(), (uint32_t)cmap_.size(), nb.blob.data(),
                                                 nb.offsets.data(), unk_id_, &n_barcodes, &names.buf, &name_offsets.buf, &offs.buf,
                                                 &ids.buf),
                   "gtgpu_tokenize_fragments_file");
-        }
     }
     const char* blob = (const char*)gtgpu_buf_data(names.buf);
     const uint64_t* noff = (const uint64_t*)gtgpu_buf_data(name_offsets.buf);
@@ -990,18 +994,8 @@ std::vector<std::pair<std::string, std::map<uint32_t, uint32_t>>> barcode_scorin
     return out;
 }
 
-// Device parse of one fragment file: a bgzip'ed file goes to the device inflater (gz_members_for_device), any other file is
-// read by read_file_bytes (a single-member gzip is inflated by zlib on the host).  Device errors are prefixed with the path.
+// Device parse of one fragment file (FileBytes).  Device errors are prefixed with the path.
 namespace {
-struct FragmentBytes {
-    std::string raw, text;
-    std::vector<uint64_t> members;
-    bool gz = false;
-    explicit FragmentBytes(const std::string& path) {
-        gz = gz_members_for_device(path, raw, members);
-        if (!gz) text = read_file_bytes(path);
-    }
-};
 void check_file(int32_t status, const std::string& path) {
     if (status != GTGPU_OK) throw Error(path + ": " + gtgpu_last_error());
 }
@@ -1016,7 +1010,7 @@ CountMatrix region_scoring_from_fragments_device(const std::vector<std::string>&
     m.data.assign(m.rows * m.cols, 0);
     for (size_t f = 0; f < fragment_files.size(); ++f) {
         const std::string& path = fragment_files[f];
-        FragmentBytes fb(path);
+        FileBytes fb(path);
         uint32_t* row = m.data.data() + f * m.cols;
         if (fb.gz)
             check_file(gtgpu_score_matrix_gz(consensus.index(), fb.members.size() - 1, (const uint8_t*)fb.raw.data(), fb.members.data(),
@@ -1033,7 +1027,7 @@ CountMatrix region_scoring_from_fragments_device(const std::vector<std::string>&
 std::vector<std::pair<std::string, std::map<uint32_t, uint32_t>>> barcode_scoring_from_fragments_device(const std::string& fragment_file,
                                                                                                         const ConsensusSet& consensus) {
     NameBlob nb(consensus.chroms());
-    FragmentBytes fb(fragment_file);
+    FileBytes fb(fragment_file);
     uint32_t n_barcodes = 0;
     PinnedResult names, name_offsets, offsets, peaks, counts;
     if (fb.gz)
