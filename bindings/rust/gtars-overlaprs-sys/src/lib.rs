@@ -67,6 +67,19 @@ extern "C" {
     pub fn gtgpu_tokenize_bed_files_gz(index: *mut gtgpu_index, n_files: u64, file_members: *const u64, n_members: u64, gz: *const u8,
                                        member_offsets: *const u64, n_names: u32, names: *const u8, name_offsets: *const u32,
                                        unk_id: u32, out_file_token_offsets: *mut u64, out_ids: *mut *mut gtgpu_buf) -> i32;
+    /// MultiChromOverlapper::{count_overlaps, any_overlaps, find_overlaps_regions, subset_by} / IndexedRegionSet::{find_overlaps,
+    /// subset_by_overlaps} of RegionSet::try_from(file f) for every file of a batch in one device pass (mode GTGPU_OVERLAPS_*);
+    /// out_file_queries (n_files + 1) counts every file's region lines, *out_offsets / *out_values as the header describes.
+    pub fn gtgpu_overlaps_bed_files(index: *mut gtgpu_index, mode: i32, n_files: u64, text: *const c_char, file_offsets: *const u64,
+                                    n_names: u32, names: *const u8, name_offsets: *const u32, min_overlap: i32, n_keys: u64,
+                                    keys: *const u32, out_file_queries: *mut u64, out_offsets: *mut *mut gtgpu_buf,
+                                    out_values: *mut *mut gtgpu_buf) -> i32;
+    /// The same from gzip members: file f = members [file_members[f], file_members[f + 1]) of gz / member_offsets.
+    pub fn gtgpu_overlaps_bed_files_gz(index: *mut gtgpu_index, mode: i32, n_files: u64, file_members: *const u64, n_members: u64,
+                                       gz: *const u8, member_offsets: *const u64, n_names: u32, names: *const u8,
+                                       name_offsets: *const u32, min_overlap: i32, n_keys: u64, keys: *const u32,
+                                       out_file_queries: *mut u64, out_offsets: *mut *mut gtgpu_buf,
+                                       out_values: *mut *mut gtgpu_buf) -> i32;
     pub fn gtgpu_tokenize_fragments_text(index: *mut gtgpu_index, text: *const u8, n_bytes: u64, n_names: u32, names: *const u8,
                                          name_offsets: *const u32, unk_id: u32, out_n_barcodes: *mut u32,
                                          out_barcode_spans: *mut *mut gtgpu_buf, out_barcode_offsets: *mut *mut gtgpu_buf,

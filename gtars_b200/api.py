@@ -69,6 +69,10 @@ def lib():
             "gth_lola_contingency": (C.c_int, [vp, u64, vp, vp, i32, vp]),
             "gth_igd_count_bed_files": (C.c_int, [vp, u64, vp, i32, C.c_int, vp, vp]),
             "gth_lola_contingency_bed_files": (C.c_int, [vp, u64, vp, cp, i32, vp]),
+            "gth_mco_overlaps_bed_files": (vp, [vp, u64, vp, C.c_int, i32]), "gth_irs_find_bed_files": (vp, [vp, u64, vp, i32]),
+            "gth_overlaps_free": (None, [vp]), "gth_overlaps_len": (u64, [vp, C.c_int]), "gth_overlaps_data": (vp, [vp, C.c_int]),
+            "gth_mco_subset_by_bed_files": (C.c_int, [vp, u64, vp, i32, vp]),
+            "gth_irs_subset_by_overlaps_bed_files": (C.c_int, [vp, u64, vp, i32, vp]),
         }
         for name, (res, args) in sig.items():
             fn = getattr(L, name)
@@ -175,6 +179,53 @@ def _take_lists(h, named=False):
         L.gth_lists_free(h)
 
 
+def _paths_arg(paths):
+    enc = [os.fsencode(p) for p in paths]
+    return enc, (C.c_char_p * max(len(enc), 1))(*enc)
+
+
+_OVERLAPS_COUNT, _OVERLAPS_ANY, _OVERLAPS_FIND = 0, 1, 2  # GTGPU_OVERLAPS_* of include/gtars_gpu.h
+
+
+def _take_overlaps(h):
+    """(file_queries, offsets, values, flags) of a gth_overlaps handle as NumPy arrays: one copy each, no per-element work."""
+    L = lib()
+    if not h:
+        _fail()
+    try:
+        out = []
+        for which, dtype in enumerate((np.uint64, np.uint64, np.uint32, np.uint8)):
+            a = np.empty(L.gth_overlaps_len(h, which), dtype=dtype)
+            if len(a):
+                C.memmove(a.ctypes.data, L.gth_overlaps_data(h, which), a.nbytes)
+            out.append(a)
+        return out
+    finally:
+        L.gth_overlaps_free(h)
+
+
+def _per_file(values, file_queries):
+    """values split into one array view per file"""
+    return np.split(values, file_queries[1:-1].astype(np.int64)) if len(file_queries) > 1 else []
+
+
+def _per_file_hits(file_queries, offsets, vals):
+    """per file (offsets from 0, vals): the file's queries' slice of a flat per-query find result"""
+    out = []
+    for f in range(len(file_queries) - 1):
+        o = offsets[int(file_queries[f]):int(file_queries[f + 1]) + 1]
+        out.append((o - o[0], vals[int(o[0]):int(o[-1])]))
+    return out
+
+
+def _subset_sets(fn, h, paths, min_overlap):
+    enc, arr = _paths_arg(paths)
+    out = (C.c_void_p * max(len(enc), 1))()
+    if fn(h, len(enc), arr, min_overlap, out):
+        _fail()
+    return [RegionSet._wrap(out[f]) for f in range(len(enc))]
+
+
 class MultiChromOverlapper:
     """gtars_overlaprs::MultiChromOverlapper over a RegionSet (val = index of the region in the source)."""
 
@@ -224,6 +275,30 @@ class MultiChromOverlapper:
         if not h:
             _fail()
         return RegionSet._wrap(h)
+
+    # ---- a batch of BED files in one device pass: element f equals the method above on RegionSet(paths[f]) ----------------
+    def _bed_files(self, paths, mode, min_overlap):
+        enc, arr = _paths_arg(paths)
+        return _take_overlaps(lib().gth_mco_overlaps_bed_files(self._h, len(enc), arr, mode, self._m(min_overlap)))
+
+    def count_overlaps_bed_files(self, paths, min_overlap=None):
+        """Per file a uint32 array: count_overlaps(RegionSet(path)), every file parsed, sorted and counted on the device."""
+        fq, _, vals, _ = self._bed_files(paths, _OVERLAPS_COUNT, min_overlap)
+        return _per_file(vals, fq)
+
+    def any_overlaps_bed_files(self, paths, min_overlap=None):
+        """Per file a bool array: any_overlaps(RegionSet(path))."""
+        fq, _, _, flags = self._bed_files(paths, _OVERLAPS_ANY, min_overlap)
+        return _per_file(flags.astype(bool), fq)
+
+    def find_overlaps_bed_files(self, paths, min_overlap=None):
+        """Per file (offsets, vals): query i of RegionSet(path) hits vals[offsets[i]:offsets[i + 1]], in find_overlaps' order."""
+        fq, off, vals, _ = self._bed_files(paths, _OVERLAPS_FIND, min_overlap)
+        return _per_file_hits(fq, off, vals)
+
+    def subset_by_bed_files(self, paths, min_overlap=None):
+        """Per file subset_by(RegionSet(path)), the distinct hit regions reduced on the device."""
+        return _subset_sets(lib().gth_mco_subset_by_bed_files, self._h, paths, self._m(min_overlap))
 
 
 def parse_bed_file(path, chrom_names):
@@ -288,6 +363,16 @@ class IndexedRegionSet:
 
     def intersect_all(self, query):
         return self.subset_by_overlaps(query, None)
+
+    def find_overlaps_bed_files(self, paths, min_overlap=None):
+        """Per file (offsets, vals): find_overlaps(RegionSet(path)) flattened, every query's indices sorted and de-duplicated."""
+        enc, arr = _paths_arg(paths)
+        fq, off, vals, _ = _take_overlaps(lib().gth_irs_find_bed_files(self._h, len(enc), arr, MultiChromOverlapper._m(min_overlap)))
+        return _per_file_hits(fq, off, vals)
+
+    def subset_by_overlaps_bed_files(self, paths, min_overlap=None):
+        """Per file subset_by_overlaps(RegionSet(path))."""
+        return _subset_sets(lib().gth_irs_subset_by_overlaps_bed_files, self._h, paths, MultiChromOverlapper._m(min_overlap))
 
     def count_overlaps(self, query, min_overlap=None):
         q = _as_rs(query)

@@ -325,7 +325,7 @@ int32_t launch_unk_expand(gtgpu_ctx* ctx, uint64_t n_files, const uint64_t* d_ra
 // ids land in scratch SC_OUT_IDS (*d_ids), *total_out is their number.  d_offsets / d_file_tok may be null.
 int32_t fused_find_all(gtgpu_index* ix, uint64_t nq, uint64_t n_files, const uint64_t* d_qfo, const uint32_t* d_qc,
                        const uint32_t* d_qs, const uint32_t* d_qe, uint64_t* d_offsets, uint64_t* d_file_tok,
-                       uint32_t** d_ids, uint64_t* total_out);
+                       uint32_t** d_ids, uint64_t* total_out, int32_t min_overlap = 0);
 
 // fragments.cu: tokenize_fragment_file over device-resident fragments with dense barcode ids (caller holds ctx->mu)
 int32_t tokenize_fragments_core(gtgpu_index* ix, uint64_t n, const uint32_t* d_chr, const uint32_t* d_start, const uint32_t* d_end,

@@ -18,6 +18,7 @@
 #include <cstring>
 #include <numeric>
 #include <string>
+#include <string_view>
 #include <thread>
 #include <vector>
 
@@ -1135,15 +1136,16 @@ __global__ void ingest_map_names_kernel(uint32_t n_names, const char* __restrict
     }
 }
 
-__global__ void ingest_remap_chr_kernel(uint64_t n, const uint32_t* __restrict__ map, uint32_t* __restrict__ chr) {
+// out[i] = map[in[i]] (in may be out)
+__global__ void ingest_remap_chr_kernel(uint64_t n, const uint32_t* __restrict__ map, const uint32_t* in, uint32_t* out) {
     const uint64_t stride = (uint64_t)gridDim.x * blockDim.x;
-    for (uint64_t i = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += stride) chr[i] = map[chr[i]];
+    for (uint64_t i = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += stride) out[i] = map[in[i]];
 }
 
-int32_t parse_bed_queries_locked(gtgpu_ctx* ctx, const Text& t, uint32_t n_names, const char* names, const uint32_t* name_offsets,
-                                 bool with_rank, const std::string& who, BedFilesRecords* r, NameTable* nt) {
-    GT_TRY(parse_bed_files_locked(ctx, t, who, r));
-    if (r->n == 0) return GTGPU_OK;
+// The r->n records' discovered name ids in_chr -> the caller's ids in out_chr (r->chr, or any other column of the records).
+static int32_t map_query_names_locked(gtgpu_ctx* ctx, const BedFilesRecords* r, uint32_t n_names, const char* names,
+                                      const uint32_t* name_offsets, bool with_rank, NameTable* nt, const uint32_t* in_chr,
+                                      uint32_t* out_chr) {
     cudaStream_t st = ctx->stream;
     GT_TRY(upload_name_table(ctx, n_names, names, name_offsets, nt, with_rank));  // scratch SC_SET_ID
     const uint64_t blob_bytes = r->names->len;
@@ -1155,11 +1157,18 @@ int32_t parse_bed_queries_locked(gtgpu_ctx* ctx, const Text& t, uint32_t n_names
     GT_CUDA(cudaMemcpyAsync(d_offs.ptr, r->name_offsets->block.ptr, ((uint64_t)r->n_names + 1) * 8, cudaMemcpyHostToDevice, st));
     ingest_map_names_kernel<<<grid_for(ctx, r->n_names), 256, 0, st>>>(r->n_names, (const char*)d_blob.ptr,
                                                                      (const unsigned long long*)d_offs.ptr, *nt, d_map.u32());
-    ingest_remap_chr_kernel<<<grid_for(ctx, r->n), 256, 0, st>>>(r->n, d_map.u32(), r->chr.u32());
+    ingest_remap_chr_kernel<<<grid_for(ctx, r->n), 256, 0, st>>>(r->n, d_map.u32(), in_chr, out_chr);
     ctx->launches += 2;
     GT_CUDA(cudaGetLastError());
     GT_CUDA(cudaStreamSynchronize(st));  // the map is freed here, and a later call may reuse the name table's scratch
     return GTGPU_OK;
+}
+
+int32_t parse_bed_queries_locked(gtgpu_ctx* ctx, const Text& t, uint32_t n_names, const char* names, const uint32_t* name_offsets,
+                                 bool with_rank, const std::string& who, BedFilesRecords* r, NameTable* nt) {
+    GT_TRY(parse_bed_files_locked(ctx, t, who, r));
+    if (r->n == 0) return GTGPU_OK;
+    return map_query_names_locked(ctx, r, n_names, names, name_offsets, with_rank, nt, r->chr.u32(), r->chr.u32());
 }
 
 // ---- a batch of BED files tokenized in one pass: parse, per-file RegionSet::sort, fused find, [unk] rule ----------------------
@@ -1226,6 +1235,198 @@ static int32_t tokenize_bed_locked(gtgpu_index* ix, const Text& t, uint32_t n_na
     return GTGPU_OK;
 }
 
+// ---- a batch of BED files against an overlap index: count / any / find / subset per file -------------------------------------
+// Per-query outputs make the query order visible, and RegionSet::try_from sorts by (chromosome STRING, start) over every name of
+// the file, names the index lacks included (region_set.rs:502-505).  So the records are sorted while their chr column still
+// holds the names discovered in the files, ranked here by their bytes, and only then mapped to the caller's ids.
+
+// hit i of the fused find's per-file runs (file_hits: n_files + 1 raw offsets): its key (keys[val], or val) and its file.
+// fold: one word file << key_bits | key for a single radix pass; otherwise the key, with the file as the pair's value.
+__global__ void overlaps_subset_keys_kernel(uint64_t total, const uint32_t* __restrict__ ids, const uint32_t* __restrict__ keys,
+                                            uint64_t n_files, const unsigned long long* __restrict__ file_hits, int key_bits, bool fold,
+                                            uint32_t* __restrict__ k, uint32_t* __restrict__ v) {
+    const uint64_t stride = (uint64_t)gridDim.x * blockDim.x;
+    for (uint64_t i = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x; i < total; i += stride) {
+        const uint32_t key = keys ? keys[ids[i]] : ids[i];
+        uint64_t lo = 0, hi = n_files;  // the last file whose hits start at or before i (files without hits start where the next does)
+        while (hi - lo > 1) {
+            const uint64_t mid = (lo + hi) >> 1;
+            if (file_hits[mid] <= i) lo = mid;
+            else hi = mid;
+        }
+        const uint32_t f = (uint32_t)lo;
+        k[i] = fold ? f << key_bits | key : key;
+        v[i] = f;
+    }
+}
+
+// 1 where a new (file, key) starts in the sorted hits (file == nullptr: key holds the folded words)
+__global__ void overlaps_subset_heads_kernel(uint64_t n, const uint32_t* __restrict__ key, const uint32_t* __restrict__ file,
+                                             uint32_t* __restrict__ head) {
+    const uint64_t stride = (uint64_t)gridDim.x * blockDim.x;
+    for (uint64_t i = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += stride)
+        head[i] = i == 0 || key[i] != key[i - 1] || (file && file[i] != file[i - 1]);
+}
+
+// the distinct (file, key) pairs at their scanned positions: keys to out_key, files to out_file (for the per-file offsets)
+__global__ void overlaps_subset_unique_kernel(uint64_t n, const uint32_t* __restrict__ key, const uint32_t* __restrict__ file,
+                                              const uint32_t* __restrict__ head, const uint32_t* __restrict__ pos, int key_bits,
+                                              uint32_t* __restrict__ out_key, uint32_t* __restrict__ out_file) {
+    const uint64_t stride = (uint64_t)gridDim.x * blockDim.x;
+    for (uint64_t i = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += stride)
+        if (head[i]) {
+            const uint32_t q = pos[i], w = key[i];
+            out_key[q] = file ? w : w & ((1u << key_bits) - 1u);
+            out_file[q] = file ? file[i] : w >> key_bits;
+        }
+}
+
+// ranks of the discovered names in byte order (Rust's String order)
+static std::vector<uint32_t> name_byte_ranks(const BedFilesRecords& r) {
+    const char* blob = (const char*)r.names->block.ptr;
+    const uint64_t* off = (const uint64_t*)r.name_offsets->block.ptr;
+    std::vector<uint32_t> by_name(r.n_names), rank(r.n_names);
+    std::iota(by_name.begin(), by_name.end(), 0u);
+    auto name = [&](uint32_t i) { return std::string_view(blob + off[i], off[i + 1] - off[i]); };
+    std::sort(by_name.begin(), by_name.end(), [&](uint32_t a, uint32_t b) { return name(a) < name(b); });  // names are distinct
+    for (uint32_t k = 0; k < r.n_names; ++k) rank[by_name[k]] = k;
+    return rank;
+}
+
+// SUBSET: the ascending distinct keys of every file's hits.  The total hits (which can exceed the queries many times) size the
+// scratch; they are sorted by (file, key) in one radix pass when both fit 32 bits, else by key and then by file.
+static int32_t subset_reduce_locked(gtgpu_index* ix, uint64_t n_files, const uint32_t* d_ids, uint64_t total, const uint64_t* d_file_hits,
+                                    const uint32_t* d_keys, uint32_t max_key, const std::string& who, BufPtr* out_offsets,
+                                    BufPtr* out_values) {
+    gtgpu_ctx* ctx = ix->ctx;
+    cudaStream_t st = ctx->stream;
+    if (total >= 0xFFFFFFFFull) return fail(GTGPU_ERR_UNSUPPORTED, who + ": 2^32 - 1 hits or more in one subset call");
+    uint64_t* d_offs;
+    uint32_t *out_key = nullptr, n_distinct = 0;
+    GT_TRY(ctx->scratch_get(SC_FILE_TOK2, (n_files + 1) * 8, (void**)&d_offs));
+    if (total == 0) {
+        GT_CUDA(cudaMemsetAsync(d_offs, 0, (n_files + 1) * 8, st));
+    } else {
+        const int key_bits = bits_for_value(max_key), file_bits = bits_for_value(n_files - 1);
+        const bool fold = key_bits + file_bits <= 32;
+        uint32_t *k_a, *v_a, *k_b, *v_b, *head, *pos, *out_file;
+        void* d_tmp;
+        const size_t b = (size_t)total * 4;
+        GT_TRY(ctx->scratch_get(SC_ING_0, b, (void**)&k_a));
+        GT_TRY(ctx->scratch_get(SC_ING_1, b, (void**)&v_a));
+        GT_TRY(ctx->scratch_get(SC_ING_2, b, (void**)&k_b));
+        GT_TRY(ctx->scratch_get(SC_ING_3, b, (void**)&v_b));
+        GT_TRY(ctx->scratch_get(SC_ING_4, b, (void**)&head));
+        GT_TRY(ctx->scratch_get(SC_ING_5, b, (void**)&pos));
+        GT_TRY(ctx->scratch_get(SC_ING_6, b, (void**)&out_file));
+        GT_TRY(ctx->scratch_get(SC_OUT_IDS2, b, (void**)&out_key));
+        GT_TRY(ctx->scratch_get(SC_IN3_START, std::max(radix_sort_temp_bytes(total), exclusive_scan_temp_bytes(total, 4)), &d_tmp));
+        overlaps_subset_keys_kernel<<<grid_for(ctx, total), 256, 0, st>>>(total, d_ids, d_keys, n_files,
+                                                                        (const unsigned long long*)d_file_hits, key_bits, fold, k_a, v_a);
+        ctx->launches++;
+        int in_b = 0;
+        GT_TRY(radix_sort_pairs(ctx, total, k_a, v_a, k_b, v_b, fold ? key_bits + file_bits : key_bits, d_tmp, &in_b));
+        if (in_b) { std::swap(k_a, k_b); std::swap(v_a, v_b); }
+        const uint32_t *s_key = k_a, *s_file = nullptr;
+        if (!fold) {  // stable by file: the files are the keys of this pass
+            GT_TRY(radix_sort_pairs(ctx, total, v_a, k_a, v_b, k_b, file_bits, d_tmp, &in_b));
+            s_key = in_b ? k_b : k_a;
+            s_file = in_b ? v_b : v_a;
+        }
+        overlaps_subset_heads_kernel<<<grid_for(ctx, total), 256, 0, st>>>(total, s_key, s_file, head);
+        ctx->launches++;
+        GT_TRY(exclusive_scan<uint32_t>(ctx, head, pos, total, d_tmp));
+        overlaps_subset_unique_kernel<<<grid_for(ctx, total), 256, 0, st>>>(total, s_key, s_file, head, pos, key_bits, out_key, out_file);
+        ctx->launches++;
+        uint32_t tail[2];
+        GT_CUDA(cudaMemcpyAsync(&tail[0], pos + total - 1, 4, cudaMemcpyDeviceToHost, st));
+        GT_CUDA(cudaMemcpyAsync(&tail[1], head + total - 1, 4, cudaMemcpyDeviceToHost, st));
+        GT_CUDA(cudaStreamSynchronize(st));
+        n_distinct = tail[0] + tail[1];
+        ingest_file_record_offsets_kernel<<<grid_for(ctx, n_files + 1), 256, 0, st>>>(n_files, out_file, n_distinct,
+                                                                                   (unsigned long long*)d_offs);
+        ctx->launches++;
+        GT_CUDA(cudaGetLastError());
+    }
+    GT_TRY(buf_from_device(ctx, d_offs, n_files + 1, 8, st, out_offsets));
+    const int32_t s = buf_from_device(ctx, out_key, n_distinct, 4, st, out_values);
+    const cudaError_t e = cudaStreamSynchronize(st);
+    GT_TRY(s);
+    if (e != cudaSuccess) return fail(GTGPU_ERR_CUDA, who + ": D2H: " + cudaGetErrorString(e));
+    return GTGPU_OK;
+}
+
+// gtgpu_overlaps_bed_files on t.n_files > 0 files.  The caller holds ctx->mu.
+static int32_t overlaps_bed_files_locked(gtgpu_index* ix, const Text& t, int32_t mode, uint32_t n_names, const char* names,
+                                         const uint32_t* name_offsets, int32_t min_overlap, uint64_t n_keys, const uint32_t* keys,
+                                         const std::string& who, uint64_t* out_file_queries, BufPtr* out_offsets, BufPtr* out_values) {
+    gtgpu_ctx* ctx = ix->ctx;
+    cudaStream_t st = ctx->stream;
+    const uint64_t n_files = t.n_files;
+    BedFilesRecords r;
+    GT_TRY(parse_bed_files_locked(ctx, t, who, &r));
+    const uint32_t n = (uint32_t)r.n;  // parse_bed_files_locked allows fewer than 2^32 - 1 records
+    // ---- per file, stable by (name bytes, start); then the names in the caller's ids (into r.chr) ------------------------------
+    // The sorted start / end may lie in scratch SC_ING_2 / SC_ING_3 (sort_regions_locked), which nothing touches before the
+    // count or the fused find has read them.
+    const uint32_t *q_chr = r.chr.u32(), *q_start = r.start.u32(), *q_end = r.end.u32();
+    {
+        const std::vector<uint32_t> rank = name_byte_ranks(r);
+        DevMem d_rank;
+        GT_TRY(d_rank.reserve((size_t)r.n_names * 4, 0, st));
+        GT_CUDA(cudaMemcpyAsync(d_rank.ptr, rank.data(), (size_t)r.n_names * 4, cudaMemcpyHostToDevice, st));
+        NameTable by_bytes{};
+        by_bytes.n_names = r.n_names;
+        by_bytes.rank = d_rank.u32();
+        GT_TRY(sort_regions_locked(ctx, n, by_bytes, r.n_names, r.file.u32(), n_files, &q_chr, &q_start, &q_end));
+        GT_CUDA(cudaStreamSynchronize(st));  // the ranks are freed here
+        NameTable nt{};
+        GT_TRY(map_query_names_locked(ctx, &r, n_names, names, name_offsets, false, &nt, q_chr, r.chr.u32()));
+        q_chr = r.chr.u32();
+    }
+    std::copy(r.file_offsets.begin(), r.file_offsets.end(), out_file_queries);
+    const int32_t m = min_overlap > 1 ? min_overlap : 0;  // the reference filters only when min_overlap > 1
+    if (mode == GTGPU_OVERLAPS_COUNT || mode == GTGPU_OVERLAPS_ANY) {
+        const size_t elem = mode == GTGPU_OVERLAPS_COUNT ? 4 : 1;
+        void* d_out;
+        GT_TRY(ctx->scratch_get(SC_COUNTS, (size_t)n * elem, &d_out));
+        GT_TRY(launch_count(ix, n, q_chr, q_start, q_end, m, mode == GTGPU_OVERLAPS_COUNT ? COUNT_U32 : COUNT_ANY_U8, d_out));
+        const int32_t s = buf_from_device(ctx, d_out, n, (uint32_t)elem, st, out_values);
+        const cudaError_t e = cudaStreamSynchronize(st);
+        GT_TRY(s);
+        if (e != cudaSuccess) return fail(GTGPU_ERR_CUDA, who + ": " + cudaGetErrorString(e));
+        return GTGPU_OK;
+    }
+    uint32_t* d_ids = nullptr;
+    uint64_t total = 0;
+    if (mode == GTGPU_OVERLAPS_FIND) {
+        uint64_t* d_offsets;
+        GT_TRY(ctx->scratch_get(SC_OUT_OFFS, ((uint64_t)n + 1) * 8, (void**)&d_offsets));
+        GT_TRY(fused_find_all(ix, n, 0, nullptr, q_chr, q_start, q_end, d_offsets, nullptr, &d_ids, &total, m));  // synchronises
+        GT_TRY(buf_from_device(ctx, d_offsets, (uint64_t)n + 1, 8, st, out_offsets));
+        const int32_t s = buf_from_device(ctx, d_ids, total, 4, st, out_values);
+        const cudaError_t e = cudaStreamSynchronize(st);
+        GT_TRY(s);
+        if (e != cudaSuccess) return fail(GTGPU_ERR_CUDA, who + ": D2H: " + cudaGetErrorString(e));
+        return GTGPU_OK;
+    }
+    // ---- SUBSET ----------------------------------------------------------------------------------------------------------------
+    uint32_t max_key = ix->max_val;
+    DevMem d_keys;
+    if (keys) {
+        max_key = n_keys ? *std::max_element(keys, keys + n_keys) : 0u;
+        GT_TRY(d_keys.reserve(n_keys * 4, 0, st));
+        GT_CUDA(cudaMemcpyAsync(d_keys.ptr, keys, n_keys * 4, cudaMemcpyHostToDevice, st));
+    }
+    uint64_t *d_fo, *d_file_hits;
+    GT_TRY(ctx->scratch_get(SC_FILE_OFFS, (n_files + 1) * 8, (void**)&d_fo));
+    GT_TRY(ctx->scratch_get(SC_FILE_TOK, (n_files + 1) * 8, (void**)&d_file_hits));
+    GT_CUDA(cudaMemcpyAsync(d_fo, r.file_offsets.data(), (n_files + 1) * 8, cudaMemcpyHostToDevice, st));
+    GT_TRY(fused_find_all(ix, n, n_files, d_fo, q_chr, q_start, q_end, nullptr, d_file_hits, &d_ids, &total, m));  // synchronises
+    return subset_reduce_locked(ix, n_files, d_ids, total, d_file_hits, keys ? d_keys.u32() : nullptr, max_key, who, out_offsets,
+                                out_values);
+}
+
 // ---- the entry points: each plain-text / gzip pair shares one body ------------------------------------------------------------
 // A body checks its arguments, takes ctx->mu, opens the text (open_text_locked: gzip members are inflated whole into device
 // memory) and parses it where it is.  `who` is the entry point's name without "gtgpu_".
@@ -1261,6 +1462,40 @@ static int32_t tokenize_bed_files_text(gtgpu_index* ix, const TextIn& in, const 
         GT_TRY(tokenize_bed_files_locked(ix, t, n_names, names, name_offsets, unk_id, who, out_file_token_offsets, &ids));
     }
     *out_ids = ids.release();
+    return GTGPU_OK;
+}
+
+static int32_t overlaps_bed_files_text(gtgpu_index* ix, const TextIn& in, const char* who, int32_t mode, uint32_t n_names,
+                                       const char* names, const uint32_t* name_offsets, int32_t min_overlap, uint64_t n_keys,
+                                       const uint32_t* keys, uint64_t* out_file_queries, gtgpu_buf** out_offsets, gtgpu_buf** out_values) {
+    const bool per_query = mode == GTGPU_OVERLAPS_COUNT || mode == GTGPU_OVERLAPS_ANY;
+    if (mode < GTGPU_OVERLAPS_COUNT || mode > GTGPU_OVERLAPS_SUBSET) return fail(GTGPU_ERR_INVALID, std::string(who) + ": unknown mode");
+    if (!ix || !out_file_queries || !out_values || (!per_query && !out_offsets) || (n_names && (!names || !name_offsets)) ||
+        (n_keys && !keys))
+        return fail(GTGPU_ERR_INVALID, std::string(who) + ": null argument");
+    if (mode == GTGPU_OVERLAPS_SUBSET && keys && n_keys <= ix->max_val)
+        return fail(GTGPU_ERR_INVALID, std::string(who) + ": keys must have an entry for every val of the index (n_keys > " +
+                                           std::to_string(ix->max_val) + ")");
+    GT_TRY(in.check(who));
+    gtgpu_ctx* ctx = ix->ctx;
+    std::lock_guard<std::mutex> lk(ctx->mu);
+    GT_CUDA(cudaSetDevice(ctx->device));
+    BufPtr offsets, values;
+    if (in.n_files == 0) {  // the offsets are [0] and the buffers empty
+        out_file_queries[0] = 0;
+        GT_TRY(buf_new(ctx, 0, mode == GTGPU_OVERLAPS_ANY ? 1 : 4, &values));
+        if (!per_query) {
+            GT_TRY(buf_new(ctx, 1, 8, &offsets));
+            *reinterpret_cast<uint64_t*>(offsets->block.ptr) = 0;
+        }
+    } else {
+        Text t;
+        GT_TRY(open_text_locked(ctx, in, who, &t));
+        GT_TRY(overlaps_bed_files_locked(ix, t, mode, n_names, names, name_offsets, min_overlap, n_keys,
+                                         mode == GTGPU_OVERLAPS_SUBSET ? keys : nullptr, who, out_file_queries, &offsets, &values));
+    }
+    if (out_offsets) *out_offsets = offsets.release();
+    *out_values = values.release();
     return GTGPU_OK;
 }
 
@@ -1390,6 +1625,23 @@ extern "C" int32_t gtgpu_tokenize_bed_files_gz(gtgpu_index* ix, uint64_t n_files
                                                gtgpu_buf** out_ids) try {
     return tokenize_bed_files_text(ix, TextIn::gzip(n_members, gz, member_offsets, n_files, file_members), "tokenize_bed_files_gz",
                                    n_names, names, name_offsets, unk_id, out_file_token_offsets, out_ids);
+} GT_CATCH
+
+extern "C" int32_t gtgpu_overlaps_bed_files(gtgpu_index* ix, int32_t mode, uint64_t n_files, const char* text, const uint64_t* file_offsets,
+                                            uint32_t n_names, const char* names, const uint32_t* name_offsets, int32_t min_overlap,
+                                            uint64_t n_keys, const uint32_t* keys, uint64_t* out_file_queries, gtgpu_buf** out_offsets,
+                                            gtgpu_buf** out_values) try {
+    return overlaps_bed_files_text(ix, TextIn::plain(text, n_files, file_offsets), "overlaps_bed_files", mode, n_names, names, name_offsets,
+                                   min_overlap, n_keys, keys, out_file_queries, out_offsets, out_values);
+} GT_CATCH
+
+extern "C" int32_t gtgpu_overlaps_bed_files_gz(gtgpu_index* ix, int32_t mode, uint64_t n_files, const uint64_t* file_members,
+                                               uint64_t n_members, const uint8_t* gz, const uint64_t* member_offsets, uint32_t n_names,
+                                               const char* names, const uint32_t* name_offsets, int32_t min_overlap, uint64_t n_keys,
+                                               const uint32_t* keys, uint64_t* out_file_queries, gtgpu_buf** out_offsets,
+                                               gtgpu_buf** out_values) try {
+    return overlaps_bed_files_text(ix, TextIn::gzip(n_members, gz, member_offsets, n_files, file_members), "overlaps_bed_files_gz", mode,
+                                   n_names, names, name_offsets, min_overlap, n_keys, keys, out_file_queries, out_offsets, out_values);
 } GT_CATCH
 
 extern "C" int32_t gtgpu_tokenize_fragments_text(gtgpu_index* ix, const char* text, uint64_t n_bytes, uint32_t n_names,

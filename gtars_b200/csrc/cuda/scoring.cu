@@ -103,7 +103,7 @@ __global__ void score_barcode_offsets_kernel(uint32_t n_barcodes, uint64_t nnz, 
 // Returns the raw ids in SC_OUT_IDS (*d_ids) and their number.
 int32_t fused_find_all(gtgpu_index* ix, uint64_t nq, uint64_t n_files, const uint64_t* d_qfo, const uint32_t* d_qc,
                         const uint32_t* d_qs, const uint32_t* d_qe, uint64_t* d_offsets, uint64_t* d_file_tok,
-                        uint32_t** d_ids, uint64_t* total_out) {
+                        uint32_t** d_ids, uint64_t* total_out, int32_t min_overlap) {
     gtgpu_ctx* ctx = ix->ctx;
     cudaStream_t st = ctx->stream;
     void* d_ws;
@@ -114,7 +114,7 @@ int32_t fused_find_all(gtgpu_index* ix, uint64_t nq, uint64_t n_files, const uin
     for (int attempt = 0; attempt < 2; ++attempt) {
         GT_TRY(ctx->scratch_get(SC_OUT_IDS, cap * 4, (void**)d_ids));
         GT_CUDA(cudaMemsetAsync(d_misc, 0, 64, st));
-        GT_TRY(launch_fused_find(ix, nq, n_files, d_qfo, d_qc, d_qs, d_qe, 0, *d_ids, cap, d_offsets, d_file_tok, d_ws, nullptr,
+        GT_TRY(launch_fused_find(ix, nq, n_files, d_qfo, d_qc, d_qs, d_qe, min_overlap, *d_ids, cap, d_offsets, d_file_tok, d_ws, nullptr,
                                  d_misc, (uint32_t*)(d_misc + 2)));
         GT_CUDA(cudaMemcpyAsync(ctx->h_scalars, d_misc, 24, cudaMemcpyDeviceToHost, st));
         GT_CUDA(cudaStreamSynchronize(st));

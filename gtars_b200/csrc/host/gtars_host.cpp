@@ -764,6 +764,138 @@ std::vector<std::vector<uint32_t>> Tokenizer::encode_bed_files(const std::vector
     return out;
 }
 
+// ---- MultiChromOverlapper / IndexedRegionSet over BED files -------------------------------------------------------------------
+void MultiChromOverlapper::coordinate_ranks() const {
+    std::call_once(ranks_once_, [&] {
+        const size_t n = source_.size();
+        std::vector<uint32_t> order(n);
+        for (uint32_t i = 0; i < n; ++i) order[i] = i;
+        auto less = [&](uint32_t a, uint32_t b) {
+            const Region &x = source_[a], &y = source_[b];
+            return x.chr != y.chr ? x.chr < y.chr : x.start != y.start ? x.start < y.start : x.end < y.end;
+        };
+        std::sort(order.begin(), order.end(), less);
+        coord_rank_.assign(n, 0);
+        rank_region_.clear();
+        for (size_t k = 0; k < n; ++k) {
+            if (k == 0 || less(order[k - 1], order[k])) rank_region_.push_back(order[k]);
+            coord_rank_[order[k]] = (uint32_t)rank_region_.size() - 1;
+        }
+    });
+}
+
+BedFilesOverlaps MultiChromOverlapper::overlaps_bed_files(const std::vector<std::string>& paths, int32_t mode, int32_t min_overlap,
+                                                          bool coordinate_keys) const {
+    const BedFilesBytes b = gather_bed_files(paths);
+    NameBlob nb(cmap_);
+    const uint32_t* keys = nullptr;
+    uint64_t n_keys = 0;
+    if (coordinate_keys && !source_.empty()) {
+        coordinate_ranks();
+        keys = coord_rank_.data();
+        n_keys = coord_rank_.size();
+    }
+    BedFilesOverlaps r;
+    r.file_queries.assign(paths.size() + 1, 0);
+    PinnedResult offs, vals;
+    int32_t status;
+    const char* fn;
+    if (b.gz) {
+        fn = "gtgpu_overlaps_bed_files_gz";
+        status = gtgpu_overlaps_bed_files_gz(index_, mode, paths.size(), b.file_members.data(), b.members.size() - 1,
+                                             (const uint8_t*)b.raw.data(), b.members.data(), (uint32_t)cmap_.size(), nb.blob.data(),
+                                             nb.offsets.data(), min_overlap, n_keys, keys, r.file_queries.data(), &offs.buf, &vals.buf);
+    } else {
+        fn = "gtgpu_overlaps_bed_files";
+        status = gtgpu_overlaps_bed_files(index_, mode, paths.size(), b.text.get(), b.file_offsets.data(), (uint32_t)cmap_.size(),
+                                          nb.blob.data(), nb.offsets.data(), min_overlap, n_keys, keys, r.file_queries.data(), &offs.buf,
+                                          &vals.buf);
+    }
+    if (status != GTGPU_OK) throw_naming_path(fn, paths);
+    if (offs.buf) {
+        const uint64_t* o = (const uint64_t*)gtgpu_buf_data(offs.buf);
+        r.offsets.assign(o, o + offs.len());
+    }
+    if (mode == GTGPU_OVERLAPS_ANY) {
+        const uint8_t* a = (const uint8_t*)gtgpu_buf_data(vals.buf);
+        r.flags.assign(a, a + vals.len());
+    } else {
+        r.values.assign(vals.data(), vals.data() + vals.len());
+    }
+    return r;
+}
+
+std::vector<std::vector<uint64_t>> MultiChromOverlapper::count_overlaps_bed_files(const std::vector<std::string>& paths,
+                                                                                  int32_t min_overlap) const {
+    const BedFilesOverlaps r = overlaps_bed_files(paths, GTGPU_OVERLAPS_COUNT, min_overlap);
+    std::vector<std::vector<uint64_t>> out(paths.size());
+    for (size_t f = 0; f < out.size(); ++f) out[f].assign(r.values.begin() + r.file_queries[f], r.values.begin() + r.file_queries[f + 1]);
+    return out;
+}
+
+std::vector<std::vector<bool>> MultiChromOverlapper::any_overlaps_bed_files(const std::vector<std::string>& paths, int32_t min_overlap) const {
+    const BedFilesOverlaps r = overlaps_bed_files(paths, GTGPU_OVERLAPS_ANY, min_overlap);
+    std::vector<std::vector<bool>> out(paths.size());
+    for (size_t f = 0; f < out.size(); ++f) out[f].assign(r.flags.begin() + r.file_queries[f], r.flags.begin() + r.file_queries[f + 1]);
+    return out;
+}
+
+// per file, per query: the hits of a flat FIND result
+static std::vector<std::vector<std::vector<uint32_t>>> per_file_hits(const BedFilesOverlaps& r) {
+    std::vector<std::vector<std::vector<uint32_t>>> out(r.file_queries.size() - 1);
+    for (size_t f = 0; f < out.size(); ++f)
+        for (uint64_t q = r.file_queries[f]; q < r.file_queries[f + 1]; ++q)
+            out[f].emplace_back(r.values.begin() + r.offsets[q], r.values.begin() + r.offsets[q + 1]);
+    return out;
+}
+
+std::vector<std::vector<std::vector<uint32_t>>> MultiChromOverlapper::find_overlaps_indices_bed_files(const std::vector<std::string>& paths,
+                                                                                                      int32_t min_overlap) const {
+    return per_file_hits(overlaps_bed_files(paths, GTGPU_OVERLAPS_FIND, min_overlap));
+}
+
+std::vector<RegionSet> MultiChromOverlapper::subset_by_bed_files(const std::vector<std::string>& paths, int32_t min_overlap) const {
+    // the distinct coordinate ranks of a file's hits, ascending, are subset_by's BTreeSet<(String, u32, u32)> in order
+    const BedFilesOverlaps r = overlaps_bed_files(paths, GTGPU_OVERLAPS_SUBSET, min_overlap, true);
+    std::vector<RegionSet> out(paths.size());
+    for (size_t f = 0; f < out.size(); ++f)
+        for (uint64_t k = r.offsets[f]; k < r.offsets[f + 1]; ++k) {
+            const Region& s = source_[rank_region_[r.values[k]]];
+            out[f].regions.push_back(Region{s.chr, s.start, s.end, ""});
+        }
+    return out;
+}
+
+BedFilesOverlaps IndexedRegionSet::find_overlaps_bed_files_flat(const std::vector<std::string>& paths, int32_t min_overlap) const {
+    BedFilesOverlaps r = index_->overlaps_bed_files(paths, GTGPU_OVERLAPS_FIND, min_overlap);
+    // every query's indices sorted and de-duplicated in place (:256-258), the runs moved down over the removed ones
+    uint64_t w = 0;
+    for (size_t q = 0; q + 1 < r.offsets.size(); ++q) {
+        const auto a = r.values.begin() + r.offsets[q], e = r.values.begin() + r.offsets[q + 1];
+        std::sort(a, e);
+        const auto u = std::unique(a, e);
+        std::copy(a, u, r.values.begin() + w);
+        r.offsets[q] = w;
+        w += (uint64_t)(u - a);
+    }
+    r.offsets.back() = w;
+    r.values.resize(w);
+    return r;
+}
+
+std::vector<std::vector<std::vector<uint32_t>>> IndexedRegionSet::find_overlaps_bed_files(const std::vector<std::string>& paths,
+                                                                                          int32_t min_overlap) const {
+    return per_file_hits(find_overlaps_bed_files_flat(paths, min_overlap));
+}
+
+std::vector<RegionSet> IndexedRegionSet::subset_by_overlaps_bed_files(const std::vector<std::string>& paths, int32_t min_overlap) const {
+    const BedFilesOverlaps r = index_->overlaps_bed_files(paths, GTGPU_OVERLAPS_SUBSET, min_overlap);  // ascending source indices
+    std::vector<RegionSet> out(paths.size());
+    for (size_t f = 0; f < out.size(); ++f)
+        for (uint64_t k = r.offsets[f]; k < r.offsets[f + 1]; ++k) out[f].regions.push_back(source_.regions[r.values[k]]);
+    return out;
+}
+
 std::vector<std::string> Tokenizer::tokenize(const std::vector<Region>& regions) const {
     std::vector<std::string> out;
     for (uint32_t id : encode(regions)) out.push_back(id_to_first_token_.at(id));

@@ -13,6 +13,7 @@
 #include <cstdint>
 #include <map>
 #include <memory>
+#include <mutex>
 #include <stdexcept>
 #include <string>
 #include <unordered_map>
@@ -93,6 +94,15 @@ void init_gtok_file(const std::string& filename);                               
 void append_tokens_to_gtok_file(const std::string& filename, const std::vector<uint32_t>& tokens);
 
 // ---- gtars_overlaprs::MultiChromOverlapper / IndexedRegionSet ------------------------------------------------------
+// The outputs of gtgpu_overlaps_bed_files for a batch of BED files, flat: file f's queries are [file_queries[f], file_queries[f + 1])
+// in RegionSet::from_file(paths[f]) order.
+struct BedFilesOverlaps {
+    std::vector<uint64_t> file_queries;  // n_files + 1
+    std::vector<uint64_t> offsets;       // find: n + 1 per query; subset: n_files + 1 per file; count / any: empty
+    std::vector<uint32_t> values;        // count: per query; find: source indices; subset: keys (coordinate ranks or indices)
+    std::vector<uint8_t> flags;          // any: 0 / 1 per query
+};
+
 class MultiChromOverlapper {
    public:
     // RegionSet::into_multi_chrom_overlapper (multi_chrom_overlapper.rs:240-300): val = index of the region in `source`.
@@ -110,11 +120,29 @@ class MultiChromOverlapper {
     // multi_chrom_overlapper.rs:449-480: deduplicated, sorted by (chr, start, end).
     RegionSet subset_by(const RegionSet& query, int32_t min_overlap = -1) const;
 
+    // The same over a batch of BED files in ONE device pass, every file parsed, sorted and resolved there
+    // (gtgpu_overlaps_bed_files; gtgpu_overlaps_bed_files_gz when every path ends in ".gz", as Tokenizer::encode_bed_files).
+    // Element f equals the method above on RegionSet::from_file(paths[f]).  Errors name the file's path.
+    std::vector<std::vector<uint64_t>> count_overlaps_bed_files(const std::vector<std::string>& paths, int32_t min_overlap = -1) const;
+    std::vector<std::vector<bool>> any_overlaps_bed_files(const std::vector<std::string>& paths, int32_t min_overlap = -1) const;
+    std::vector<std::vector<std::vector<uint32_t>>> find_overlaps_indices_bed_files(const std::vector<std::string>& paths,
+                                                                                    int32_t min_overlap = -1) const;
+    std::vector<RegionSet> subset_by_bed_files(const std::vector<std::string>& paths, int32_t min_overlap = -1) const;
+    // gtgpu_overlaps_bed_files itself (mode: GTGPU_OVERLAPS_*).  SUBSET keys: the source regions' coordinate ranks when
+    // coordinate_keys (subset_by's (chr, start, end) set), else the source indices.
+    BedFilesOverlaps overlaps_bed_files(const std::vector<std::string>& paths, int32_t mode, int32_t min_overlap,
+                                        bool coordinate_keys = false) const;
+
    private:
     std::shared_ptr<Device> dev_;
     gtgpu_index* index_ = nullptr;
     ChromMap cmap_;
     std::vector<Region> source_;  // coordinates only, to rebuild regions from vals
+    // Per source region its rank in (chromosome, start, end) order, equal coordinates sharing one, and per rank a region that
+    // has it: computed on the first subset_by_bed_files.
+    mutable std::once_flag ranks_once_;
+    mutable std::vector<uint32_t> coord_rank_, rank_region_;
+    void coordinate_ranks() const;
 };
 
 // gtars_overlaprs::IndexedRegionSet (indexed_region_set.rs:100-263): a RegionSet plus its overlap index; the
@@ -128,6 +156,12 @@ class IndexedRegionSet {
     std::vector<uint64_t> count_overlaps(const RegionSet& query, int32_t min_overlap = -1) const;           // :234-238
     std::vector<bool> any_overlaps(const RegionSet& query, int32_t min_overlap = -1) const;                 // :240-244
     std::vector<std::vector<uint32_t>> find_overlaps(const RegionSet& query, int32_t min_overlap = -1) const;  // :246-263
+    // find_overlaps / subset_by_overlaps of RegionSet::from_file(paths[f]) for every f in ONE device pass (as
+    // MultiChromOverlapper::count_overlaps_bed_files).  The flat form has every query's indices sorted and de-duplicated.
+    std::vector<std::vector<std::vector<uint32_t>>> find_overlaps_bed_files(const std::vector<std::string>& paths,
+                                                                            int32_t min_overlap = -1) const;
+    BedFilesOverlaps find_overlaps_bed_files_flat(const std::vector<std::string>& paths, int32_t min_overlap = -1) const;
+    std::vector<RegionSet> subset_by_overlaps_bed_files(const std::vector<std::string>& paths, int32_t min_overlap = -1) const;
 
    private:
     RegionSet source_;

@@ -131,6 +131,46 @@ int gth_irs_any(void* r, void* query, int32_t min_overlap, uint8_t* out) {
     }, 1);
 }
 
+// ---- the same over BED files: flat results (one copy into the caller's arrays, no per-element conversion) ----------------------
+// gth_mco_overlaps_bed_files (mode COUNT / ANY / FIND) and gth_irs_find_bed_files return a BedFilesOverlaps handle; its arrays
+// are read with gth_overlaps_len / gth_overlaps_data, which: 0 file_queries (u64), 1 offsets (u64), 2 values (u32), 3 flags (u8).
+void* gth_mco_overlaps_bed_files(void* m, uint64_t n, const char** paths, int mode, int32_t min_overlap) {
+    return guard([&]() -> void* {
+        return new BedFilesOverlaps(
+            ((MultiChromOverlapper*)m)->overlaps_bed_files(std::vector<std::string>(paths, paths + n), mode, min_overlap));
+    }, nullptr);
+}
+void* gth_irs_find_bed_files(void* r, uint64_t n, const char** paths, int32_t min_overlap) {
+    return guard([&]() -> void* {
+        return new BedFilesOverlaps(((IndexedRegionSet*)r)->find_overlaps_bed_files_flat(std::vector<std::string>(paths, paths + n), min_overlap));
+    }, nullptr);
+}
+void gth_overlaps_free(void* h) { delete (BedFilesOverlaps*)h; }
+uint64_t gth_overlaps_len(void* h, int which) {
+    const BedFilesOverlaps& o = *(BedFilesOverlaps*)h;
+    return which == 0 ? o.file_queries.size() : which == 1 ? o.offsets.size() : which == 2 ? o.values.size() : o.flags.size();
+}
+const void* gth_overlaps_data(void* h, int which) {
+    const BedFilesOverlaps& o = *(BedFilesOverlaps*)h;
+    return which == 0 ? (const void*)o.file_queries.data() : which == 1 ? (const void*)o.offsets.data()
+                                                           : which == 2 ? (const void*)o.values.data() : (const void*)o.flags.data();
+}
+// out_sets: n RegionSet handles, one per path
+int gth_mco_subset_by_bed_files(void* m, uint64_t n, const char** paths, int32_t min_overlap, void** out_sets) {
+    return guard([&]() -> int {
+        auto sets = ((MultiChromOverlapper*)m)->subset_by_bed_files(std::vector<std::string>(paths, paths + n), min_overlap);
+        for (uint64_t f = 0; f < n; ++f) out_sets[f] = new RegionSet(std::move(sets[f]));
+        return 0;
+    }, 1);
+}
+int gth_irs_subset_by_overlaps_bed_files(void* r, uint64_t n, const char** paths, int32_t min_overlap, void** out_sets) {
+    return guard([&]() -> int {
+        auto sets = ((IndexedRegionSet*)r)->subset_by_overlaps_bed_files(std::vector<std::string>(paths, paths + n), min_overlap);
+        for (uint64_t f = 0; f < n; ++f) out_sets[f] = new RegionSet(std::move(sets[f]));
+        return 0;
+    }, 1);
+}
+
 // ---- gtars_scoring ---------------------------------------------------------------------------------------------------------------
 void* gth_consensus_new(void* dev, const char* path) {
     return guard([&]() -> void* { return new ConsensusSet(*(std::shared_ptr<Device>*)dev, std::string(path)); }, nullptr);

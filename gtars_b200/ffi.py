@@ -15,6 +15,7 @@ _PKG = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.environ.get("GTGPU_LIB") or os.path.join(_PKG, "libgtars_gpu.so")
 
 SCORE_ATAC, SCORE_CHIP = 0, 1
+OVERLAPS_COUNT, OVERLAPS_ANY, OVERLAPS_FIND, OVERLAPS_SUBSET = 0, 1, 2, 3
 KIND_BITS, KIND_AILIST = 0, 1
 UNKNOWN_CHROM = 0xFFFFFFFF
 
@@ -57,6 +58,8 @@ SIGNATURES = {
     "gtgpu_tokenize_bed": (_i32, [_vp, _vp, _u64, _u32, _vp, _vp, _u32, _vp]),
     "gtgpu_tokenize_bed_files": (_i32, [_vp, _u64, _vp, _vp, _u32, _vp, _vp, _u32, _vp, _vp]),
     "gtgpu_tokenize_bed_files_gz": (_i32, [_vp, _u64, _vp, _u64, _vp, _vp, _u32, _vp, _vp, _u32, _vp, _vp]),
+    "gtgpu_overlaps_bed_files": (_i32, [_vp, _i32, _u64, _vp, _vp, _u32, _vp, _vp, _i32, _u64, _vp, _vp, _vp, _vp]),
+    "gtgpu_overlaps_bed_files_gz": (_i32, [_vp, _i32, _u64, _vp, _u64, _vp, _vp, _u32, _vp, _vp, _i32, _u64, _vp, _vp, _vp, _vp]),
     "gtgpu_tokenize_fragments_text": (_i32, [_vp, _vp, _u64, _u32, _vp, _vp, _u32, _vp, _vp, _vp, _vp]),
     "gtgpu_gzip_members": (_i32, [_vp, _u64, _u64, _vp, _vp]),
     "gtgpu_gunzip": (_i32, [_vp, _u64, _vp, _vp, _vp, _vp]),
@@ -385,6 +388,30 @@ class Index:
         check(lib().gtgpu_tokenize_bed_files_gz(self._h, len(fm) - 1, _p(fm), len(mo) - 1, _text_ptr(gz), _p(mo), len(chrom_names),
                                                 blob, _p(offs), unk_id, _p(out_off), C.byref(h)))
         return out_off, _take(h)
+
+    def _overlaps_bed(self, mode, n_files, chrom_names, min_overlap, keys, call):
+        blob, offs = _names_blob(chrom_names)
+        k = None if keys is None else _arr(keys, np.uint32)
+        fq = np.empty(n_files + 1, dtype=np.uint64)
+        ho, hv = C.c_void_p(), C.c_void_p()
+        check(call(blob, offs, min_overlap, 0 if k is None else len(k), _p(k), _p(fq), C.byref(ho), C.byref(hv)))
+        vals = _take(hv, np.uint8 if mode == OVERLAPS_ANY else np.uint32)
+        return fq, (_take(ho, np.uint64) if ho.value else None), vals
+
+    def overlaps_bed_text(self, mode, text, file_offsets, chrom_names, min_overlap=0, keys=None):
+        """gtgpu_overlaps_bed_files: file f = text[file_offsets[f]:file_offsets[f + 1]] parsed and sorted per file on the device,
+        then counted / flagged / found / subset (mode OVERLAPS_*).  Returns (file_queries, offsets or None, values)."""
+        fo = _arr(file_offsets, np.uint64)
+        return self._overlaps_bed(mode, len(fo) - 1, chrom_names, min_overlap, keys, lambda blob, offs, m, nk, kp, fq, ho, hv:
+                                  lib().gtgpu_overlaps_bed_files(self._h, mode, len(fo) - 1, _text_ptr(text), _p(fo), len(chrom_names),
+                                                                 blob, _p(offs), m, nk, kp, fq, ho, hv))
+
+    def overlaps_bed_gz(self, mode, gz, file_members, member_offsets, chrom_names, min_overlap=0, keys=None):
+        """gtgpu_overlaps_bed_files_gz: file f = gzip members [file_members[f], file_members[f + 1]) of `gz`."""
+        fm, mo = _arr(file_members, np.uint64), _arr(member_offsets, np.uint64)
+        return self._overlaps_bed(mode, len(fm) - 1, chrom_names, min_overlap, keys, lambda blob, offs, m, nk, kp, fq, ho, hv:
+                                  lib().gtgpu_overlaps_bed_files_gz(self._h, mode, len(fm) - 1, _p(fm), len(mo) - 1, _text_ptr(gz), _p(mo),
+                                                                    len(chrom_names), blob, _p(offs), m, nk, kp, fq, ho, hv))
 
     def tokenize_fragments_text(self, text: bytes, chrom_names, unk_id, gz_member_offsets=None):
         """gtgpu_tokenize_fragments_text (or _gz when gz_member_offsets is given: `text` is then the gzip data):

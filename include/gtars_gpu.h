@@ -243,6 +243,38 @@ int32_t gtgpu_tokenize_bed_files_gz(gtgpu_index* index, uint64_t n_files, const 
                                     const uint32_t* name_offsets, uint32_t unk_id, uint64_t* out_file_token_offsets,
                                     gtgpu_buf** out_ids);
 
+/* MultiChromOverlapper::{count_overlaps, any_overlaps, find_overlaps_regions, subset_by} (multi_chrom_overlapper.rs:449-550) and
+ * IndexedRegionSet::{find_overlaps, subset_by_overlaps} (indexed_region_set.rs:201-263) of RegionSet::try_from(file f) for a batch
+ * of n_files BED files in one device pass.  Inputs, line rules, windows, the header rule per file, the limits and the errors are
+ * those of gtgpu_tokenize_bed_files / _gz ("file k, line j" for a malformed line; "file k: ... 0 regions found" for a file without
+ * a region line; GTGPU_ERR_UNSUPPORTED past 262 144 distinct names or 2^32 - 1 region lines).  Chromosome names map through the
+ * caller's table as in gtgpu_tokenize_bed; a name not in it produces no hits.
+ *  - out_file_queries (n_files + 1, caller-allocated): the cumulative region lines per file (RegionSet::len: every region line,
+ *    lines on unknown names and lines with start >= end included).
+ *  - Query i of file f is region i of RegionSet::try_from(file f): stable by (chromosome name BYTES, start) over every name of
+ *    the file, names the table lacks included (chr1 < chr10 < chr1_random < chr2); such a query has count 0 / no hits.
+ *  - min_overlap filters only when > 1 (-1, 0 and 1 give the same result).  Bits and AIList indexes; FIND keeps the backend's
+ *    hit order.
+ *  - COUNT: *out_values = one u32 per query; ANY: one u8 (0 / 1) per query; *out_offsets (when out_offsets is not NULL) is NULL.
+ *  - FIND: *out_offsets = n + 1 u64 per-query offsets (n = out_file_queries[n_files]) into *out_values, the hits' vals (u32).
+ *  - SUBSET: *out_offsets = n_files + 1 u64 per-file offsets into *out_values: per file the distinct keys[val] (keys given, n_keys
+ *    entries, n_keys > every val of the index) or vals (keys NULL) over all hits of all its queries, ascending.  With keys = the
+ *    source regions' ranks in (chromosome, start, end) order, shared by equal coordinates, that is MultiChromOverlapper::subset_by
+ *    (a BTreeSet<(String, u32, u32)>); keys NULL gives IndexedRegionSet::subset_by_overlaps (a BTreeSet<usize>).
+ *  - n_files == 0 gives out_file_queries [0], empty value buffers and, for FIND / SUBSET, offsets [0].  On a multi-device ctx the
+ *    call runs on the first device. */
+#define GTGPU_OVERLAPS_COUNT 0  /* MultiChromOverlapper::count_overlaps: u32 per query             */
+#define GTGPU_OVERLAPS_ANY 1    /* any_overlaps: u8 per query                                       */
+#define GTGPU_OVERLAPS_FIND 2   /* find: n + 1 u64 per-query offsets + u32 vals in the backend order */
+#define GTGPU_OVERLAPS_SUBSET 3 /* per file: the ascending distinct keys[val] over all its hits      */
+int32_t gtgpu_overlaps_bed_files(gtgpu_index* index, int32_t mode, uint64_t n_files, const char* text, const uint64_t* file_offsets,
+                                 uint32_t n_names, const char* names, const uint32_t* name_offsets, int32_t min_overlap, uint64_t n_keys,
+                                 const uint32_t* keys, uint64_t* out_file_queries, gtgpu_buf** out_offsets, gtgpu_buf** out_values);
+int32_t gtgpu_overlaps_bed_files_gz(gtgpu_index* index, int32_t mode, uint64_t n_files, const uint64_t* file_members, uint64_t n_members,
+                                    const uint8_t* gz, const uint64_t* member_offsets, uint32_t n_names, const char* names,
+                                    const uint32_t* name_offsets, int32_t min_overlap, uint64_t n_keys, const uint32_t* keys,
+                                    uint64_t* out_file_queries, gtgpu_buf** out_offsets, gtgpu_buf** out_values);
+
 /* tokenize_fragment_file (gtars-tokenizers/src/utils/fragments.rs:12-82) from the file's (decompressed) text: lines
  * starting with '#' are skipped, every other line needs at least five whitespace-separated fields (chr start end
  * barcode ...) with start and end accepted by str::parse::<u32>() — otherwise GTGPU_ERR_INVALID with the 0-based line
