@@ -123,6 +123,19 @@ extern "C" {
                                             out_n_barcodes: *mut u32, out_barcode_names: *mut *mut gtgpu_buf,
                                             out_barcode_name_offsets: *mut *mut gtgpu_buf, out_barcode_offsets: *mut *mut gtgpu_buf,
                                             out_ids: *mut *mut gtgpu_buf) -> i32;
+    /// count_fragments_by_barcode from the file's text: per barcode (first-appearance order) its distinct token ids ascending
+    /// (u32 tokens) and their counts (u32), indexed by n_barcodes + 1 u64 offsets.
+    pub fn gtgpu_count_fragments_file(index: *mut gtgpu_index, text: *const u8, n_bytes: u64, n_names: u32, names: *const u8,
+                                      name_offsets: *const u32, unk_id: u32, out_n_barcodes: *mut u32,
+                                      out_barcode_names: *mut *mut gtgpu_buf, out_barcode_name_offsets: *mut *mut gtgpu_buf,
+                                      out_barcode_offsets: *mut *mut gtgpu_buf, out_tokens: *mut *mut gtgpu_buf,
+                                      out_counts: *mut *mut gtgpu_buf) -> i32;
+    /// The same from the file's gzip members.
+    pub fn gtgpu_count_fragments_file_gz(index: *mut gtgpu_index, n_members: u64, gz: *const u8, member_offsets: *const u64,
+                                         n_names: u32, names: *const u8, name_offsets: *const u32, unk_id: u32,
+                                         out_n_barcodes: *mut u32, out_barcode_names: *mut *mut gtgpu_buf,
+                                         out_barcode_name_offsets: *mut *mut gtgpu_buf, out_barcode_offsets: *mut *mut gtgpu_buf,
+                                         out_tokens: *mut *mut gtgpu_buf, out_counts: *mut *mut gtgpu_buf) -> i32;
     pub fn gtgpu_score_matrix(index: *mut gtgpu_index, n_files: u64, file_offsets: *const u64, n: u64, chr: *const u32,
                               start: *const u32, end: *const u32, mode: i32, n_cols: u64, out_counts: *mut u32) -> i32;
     pub fn gtgpu_score_matrix_dev(index: *mut gtgpu_index, n_files: u64, d_file_offsets: *const u64, n: u64,

@@ -4,6 +4,7 @@
     gtars.models.Region / RegionSet     -> Region, RegionSet  (gtars-python/src/models/region_set.rs:445-481)
     gtars_overlaprs MultiChromOverlapper / IndexedRegionSet -> MultiChromOverlapper
     gtars.tokenizers.tokenize_fragment_file                 -> tokenize_fragment_file
+    gtars-tokenizers count_fragments_by_barcode             -> count_fragments_by_barcode
     gtars.lola RegionDB / run_lola (contingency counts)     -> Igd, lola_contingency, lola_contingency_from_bed_files
 
 Every batch method is one call into the C++ layer, which marshals to the C ABI of include/gtars_gpu.h; nothing here
@@ -57,6 +58,7 @@ def lib():
             "gth_tokenizer_kind": (C.c_int, [vp]), "gth_tokenizer_encode_batch": (vp, [vp, u64, vp]),
             "gth_tokenizer_fragments": (vp, [vp, cp]), "gth_tokenizer_fragments_device": (vp, [vp, cp]), "gth_tokenizer_encode_bed_file": (vp, [vp, cp]),
             "gth_tokenizer_encode_bed_files": (vp, [vp, u64, vp]),
+            "gth_tokenizer_count_fragments": (vp, [vp, cp]), "gth_tokenizer_count_fragments_device": (vp, [vp, cp]),
             "gth_parse_bed_file": (vp, [vp, cp, u64, vp]), "gth_gtok_write": (C.c_int, [cp, u64, vp, C.c_int]),
             "gth_gtok_read": (vp, [cp]),
             "gth_igd_single": (vp, [vp, vp]), "gth_igd_find_pairs": (vp, [vp, vp, i32]),
@@ -542,6 +544,15 @@ def tokenize_fragment_file(path, tokenizer: Tokenizer, device_parse: bool = Fals
     for a file of any size."""
     fn = lib().gth_tokenizer_fragments_device if device_parse else lib().gth_tokenizer_fragments
     return dict(_take_lists(fn(tokenizer._h, os.fsencode(path)), named=True))
+
+
+def count_fragments_by_barcode(path, tokenizer: Tokenizer, device_parse: bool = False) -> dict:
+    """gtars-tokenizers count_fragments_by_barcode (utils/fragments.rs:87-112): {barcode: {token id: count}}, barcodes in
+    first-appearance order; a fragment with no hit counts under the unk id.  device_parse=True parses the text, tokenizes and
+    counts on the device (gtgpu_count_fragments_file / _gz), for a file of any size."""
+    fn = lib().gth_tokenizer_count_fragments_device if device_parse else lib().gth_tokenizer_count_fragments
+    named = _take_lists(fn(tokenizer._h, os.fsencode(path)), named=True)
+    return {bc: dict(zip(flat[0::2], flat[1::2])) for bc, flat in named}
 
 
 class Igd:

@@ -326,10 +326,22 @@ int32_t launch_unk_expand(gtgpu_ctx* ctx, uint64_t n_files, const uint64_t* d_ra
 int32_t fused_find_all(gtgpu_index* ix, uint64_t nq, uint64_t n_files, const uint64_t* d_qfo, const uint32_t* d_qc,
                        const uint32_t* d_qs, const uint32_t* d_qe, uint64_t* d_offsets, uint64_t* d_file_tok,
                        uint32_t** d_ids, uint64_t* total_out, int32_t min_overlap = 0);
+// scoring.cu: `total` device (key, value) pairs -> CSR, by two stable radix sorts (values of val_bits bits, then keys < n_keys)
+// and a run-length encode.  out_key_offsets (host, n_keys + 1) index, per key, its distinct values in ascending order
+// (*out_values) and how often each occurs (*out_counts).  d_keys / d_vals are sorted in place and must lie outside the scratch
+// this takes (SC_IN2_START, SC_IN2_END, SC_IN3_*, SC_COUNTS, SC_OUT_IDS2, SC_FILE_TOK): a slot that grows is freed.  who names
+// the caller in errors.  Synchronises the ctx stream; the caller holds ctx->mu.
+int32_t reduce_pairs_csr_locked(gtgpu_ctx* ctx, uint64_t total, uint32_t* d_keys, uint32_t* d_vals, int val_bits, uint32_t n_keys,
+                                uint64_t* out_key_offsets, gtgpu_buf** out_values, gtgpu_buf** out_counts, const std::string& who);
 
 // fragments.cu: tokenize_fragment_file over device-resident fragments with dense barcode ids (caller holds ctx->mu)
 int32_t tokenize_fragments_core(gtgpu_index* ix, uint64_t n, const uint32_t* d_chr, const uint32_t* d_start, const uint32_t* d_end,
                                 uint32_t* d_bc, uint32_t n_barcodes, uint32_t unk_id, uint64_t* out_barcode_offsets, BufPtr* out_ids);
+// fragments.cu: count_fragments_by_barcode over the same input: out_barcode_offsets (host, n_barcodes + 1) index each barcode's
+// distinct token ids in ascending order (*out_tokens) and their counts (*out_counts); a fragment without a hit counts as unk_id
+int32_t count_fragments_core(gtgpu_index* ix, uint64_t n, const uint32_t* d_chr, const uint32_t* d_start, const uint32_t* d_end,
+                             const uint32_t* d_bc, uint32_t n_barcodes, uint32_t unk_id, uint64_t* out_barcode_offsets,
+                             gtgpu_buf** out_tokens, gtgpu_buf** out_counts);
 
 // sort.cu — hand-written scan / radix sort
 size_t exclusive_scan_temp_bytes(uint64_t n, size_t elem);

@@ -153,6 +153,46 @@ int32_t tokenize_fragments_core(gtgpu_index* ix, uint64_t n, const uint32_t* d_c
     return GTGPU_OK;
 }
 
+// count_fragments_by_barcode (fragments.rs:87-112): the tagged find of step 1 gives every token (hits, or unk) with its
+// barcode, step 2 tags the tokens when the lean kernel fell back, and the scoring reducer sorts the (barcode, token) pairs by
+// token, then by barcode, and run-length encodes them.  The token sort needs max(max_val, unk_id)'s bits: unk_id is usually
+// the universe's size, one bit past max_val when that size is a power of two.
+int32_t count_fragments_core(gtgpu_index* ix, uint64_t n, const uint32_t* d_chr, const uint32_t* d_start, const uint32_t* d_end,
+                             const uint32_t* d_bc, uint32_t n_barcodes, uint32_t unk_id, uint64_t* out_barcode_offsets,
+                             gtgpu_buf** out_tokens, gtgpu_buf** out_counts) {
+    gtgpu_ctx* ctx = ix->ctx;
+    uint32_t *d_tok = nullptr, *d_tag = nullptr;
+    uint64_t total = 0;
+    if (n) {
+        uint64_t *d_off, *d_misc;
+        void* d_ws;
+        GT_TRY(ctx->scratch_get(SC_OUT_OFFS, (n + 1) * 8, (void**)&d_off));
+        GT_TRY(ctx->scratch_get(SC_TILE_STATUS, fused_workspace_bytes(n), &d_ws));
+        GT_TRY(ctx->scratch_get(SC_MISC, 64, (void**)&d_misc));
+        uint64_t cap = n + n / 4 + 1024;
+        const uint32_t* tag_if = nullptr;
+        for (int attempt = 0; attempt < 2; ++attempt) {
+            if (cap >= 0xFFFFFFFFull) return fail(GTGPU_ERR_UNSUPPORTED, "count_fragments: more than 2^32-2 tokens per call");
+            // the tokens and their tags stay out of the reducer's scratch (SC_OUT_IDS, SC_IN2_CHR)
+            GT_TRY(ctx->scratch_get(SC_OUT_IDS, cap * 4, (void**)&d_tok));
+            GT_TRY(ctx->scratch_get(SC_IN2_CHR, cap * 4, (void**)&d_tag));
+            GT_TRY(fragments_group_by(ix, n, d_chr, d_start, d_end, d_bc, n_barcodes, unk_id, cap, d_tok, d_tok, d_tag, nullptr, d_off,
+                                      d_ws, nullptr, d_misc, nullptr, nullptr, 1, &tag_if));
+            GT_CUDA(cudaMemcpyAsync(ctx->h_scalars, d_misc, 24, cudaMemcpyDeviceToHost, ctx->stream));
+            GT_CUDA(cudaStreamSynchronize(ctx->stream));
+            total = ctx->h_scalars[0];
+            if ((uint32_t)ctx->h_scalars[2] != 0) return fail(GTGPU_ERR_UNSUPPORTED, "count_fragments: tile overflow");
+            if (total <= cap) break;
+            if (attempt == 1) return fail(GTGPU_ERR_CAPACITY, "count_fragments: output capacity exceeded twice");
+            cap = total;  // multi-hit universes: redo with an exact buffer
+        }
+        frag_tag_tokens_kernel<<<grid_for(ctx, n), 256, 0, ctx->stream>>>(n, d_off, d_bc, cap, d_tag, tag_if);
+        ctx->launches++;
+    }
+    return reduce_pairs_csr_locked(ctx, total, d_tag, d_tok, bits_for_value(std::max(ix->max_val, unk_id)), n_barcodes,
+                                   out_barcode_offsets, out_tokens, out_counts, "count_fragments");
+}
+
 }  // namespace gtgpu
 
 static int32_t tokenize_fragments_one(gtgpu_index* ix, uint64_t n, const uint32_t* chr, const uint32_t* start, const uint32_t* end,

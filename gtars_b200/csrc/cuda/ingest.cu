@@ -996,30 +996,34 @@ int32_t KeyTable::finish(gtgpu_ctx* ctx, uint32_t* n_kept, BufPtr* out_names, Bu
     return GTGPU_OK;
 }
 
-// tokenize_fragment_file (fragments.rs:61-82) from a fragment file's text of any size: every window is parsed and its barcodes
-// go into one KeyTable that keeps every barcode; after the last window the fragment tokenizer core runs once over the
-// accumulated fragments and their dense barcode ids.  With out_spans the barcodes come back as u32 (first byte, length) spans
-// into the text, else as names + u64 name offsets.  The caller holds ctx->mu.
+// The fragment lines of tokenize_fragment_file (fragments.rs:12-56) from a fragment file's text of any size: every window is
+// parsed and its fragments and barcodes go into *tab, a KeyTable that keeps every barcode.  The caller holds ctx->mu.
+static int32_t parse_fragment_file_locked(gtgpu_ctx* ctx, const Text& t, uint32_t n_names, const char* names, const uint32_t* name_offsets,
+                                          const std::string& who, KeyTable* tab) {
+    if (t.n_bytes == 0) return GTGPU_OK;
+    NameTable nt;
+    GT_TRY(upload_name_table(ctx, n_names, names, name_offsets, &nt));
+    return for_each_window(ctx, t, who, [&](const char* d, uint64_t nb, uint64_t byte0, uint64_t line0, uint32_t* n_lines) -> int32_t {
+        ParsedLines fp;
+        GT_TRY(parse_lines_locked(ctx, d, nb, FRAG_TOKENIZE, nt, BedFilesView{}, &fp));
+        *n_lines = fp.n_lines;
+        if (fp.bad_line != 0xFFFFFFFFu)
+            return fail(GTGPU_ERR_INVALID, who + ": Invalid fragment file detected at line: " + std::to_string(line0 + fp.bad_line));
+        if (tab->n + fp.n > 0xFFFFFFFFull) return fail(GTGPU_ERR_UNSUPPORTED, who + ": more than 2^32 - 1 fragments in one file");
+        return tab->add_window(ctx, d, byte0, fp, n_names);
+    });
+}
+
+// tokenize_fragment_file (fragments.rs:61-82) from a fragment file's text of any size: after the windowed parse the fragment
+// tokenizer core runs once over the accumulated fragments and their dense barcode ids.  With out_spans the barcodes come back
+// as u32 (first byte, length) spans into the text, else as names + u64 name offsets.  The caller holds ctx->mu.
 static int32_t tokenize_fragments_file_locked(gtgpu_index* ix, const Text& t, uint32_t n_names, const char* names,
                                               const uint32_t* name_offsets, uint32_t unk_id, const std::string& who, uint32_t* out_n_barcodes,
                                               BufPtr* out_names, BufPtr* out_name_offsets, BufPtr* out_spans, BufPtr* out_barcode_offsets,
                                               BufPtr* out_ids) {
     gtgpu_ctx* ctx = ix->ctx;
     KeyTable tab(true, out_spans != nullptr, ~0ull, who, "gtgpu_tokenize_fragments", "barcode", "barcodes");
-    if (t.n_bytes) {
-        NameTable nt;
-        GT_TRY(upload_name_table(ctx, n_names, names, name_offsets, &nt));
-        GT_TRY(for_each_window(ctx, t, who,
-                               [&](const char* d, uint64_t nb, uint64_t byte0, uint64_t line0, uint32_t* n_lines) -> int32_t {
-            ParsedLines fp;
-            GT_TRY(parse_lines_locked(ctx, d, nb, FRAG_TOKENIZE, nt, BedFilesView{}, &fp));
-            *n_lines = fp.n_lines;
-            if (fp.bad_line != 0xFFFFFFFFu)
-                return fail(GTGPU_ERR_INVALID, who + ": Invalid fragment file detected at line: " + std::to_string(line0 + fp.bad_line));
-            if (tab.n + fp.n > 0xFFFFFFFFull) return fail(GTGPU_ERR_UNSUPPORTED, who + ": more than 2^32 - 1 fragments in one file");
-            return tab.add_window(ctx, d, byte0, fp, n_names);
-        }));
-    }
+    GT_TRY(parse_fragment_file_locked(ctx, t, n_names, names, name_offsets, who, &tab));
     uint32_t n_barcodes = 0;
     BufPtr offs, ids;
     GT_TRY(tab.finish(ctx, &n_barcodes, out_names, out_name_offsets, out_spans));
@@ -1567,6 +1571,36 @@ static int32_t tokenize_fragments_names(gtgpu_index* ix, const TextIn& in, const
     return GTGPU_OK;
 }
 
+// count_fragments_by_barcode (fragments.rs:87-112) from the file's text, any size: the parse of tokenize_fragments_names, then
+// per barcode its distinct token ids and their counts.
+static int32_t count_fragments_file(gtgpu_index* ix, const TextIn& in, const char* who, uint32_t n_names, const char* names,
+                                    const uint32_t* name_offsets, uint32_t unk_id, uint32_t* out_n_barcodes,
+                                    gtgpu_buf** out_barcode_names, gtgpu_buf** out_barcode_name_offsets,
+                                    gtgpu_buf** out_barcode_offsets, gtgpu_buf** out_tokens, gtgpu_buf** out_counts) {
+    if (!ix || !out_n_barcodes || !out_barcode_names || !out_barcode_name_offsets || !out_barcode_offsets || !out_tokens || !out_counts ||
+        (n_names && (!names || !name_offsets)))
+        return fail(GTGPU_ERR_INVALID, std::string(who) + ": null argument");
+    GT_TRY(in.check(who));
+    gtgpu_ctx* ctx = ix->ctx;
+    std::lock_guard<std::mutex> lk(ctx->mu);
+    GT_CUDA(cudaSetDevice(ctx->device));
+    Text t;
+    GT_TRY(open_text_locked(ctx, in, who, &t));
+    KeyTable tab(true, false, ~0ull, who, "gtgpu_tokenize_fragments", "barcode", "barcodes");
+    GT_TRY(parse_fragment_file_locked(ctx, t, n_names, names, name_offsets, who, &tab));
+    uint32_t n_barcodes = 0;
+    BufPtr nm, no, offs;
+    GT_TRY(tab.finish(ctx, &n_barcodes, &nm, &no));
+    GT_TRY(buf_new(ctx, (uint64_t)n_barcodes + 1, 8, &offs));
+    GT_TRY(count_fragments_core(ix, tab.n, tab.chr.u32(), tab.start.u32(), tab.end.u32(), tab.id.u32(), n_barcodes, unk_id,
+                                (uint64_t*)offs->block.ptr, out_tokens, out_counts));
+    *out_n_barcodes = n_barcodes;
+    *out_barcode_names = nm.release();
+    *out_barcode_name_offsets = no.release();
+    *out_barcode_offsets = offs.release();
+    return GTGPU_OK;
+}
+
 }  // namespace gtgpu
 
 using namespace gtgpu;
@@ -1679,4 +1713,22 @@ extern "C" int32_t gtgpu_tokenize_fragments_file_gz(gtgpu_index* ix, uint64_t n_
     return tokenize_fragments_names(ix, TextIn::gzip(n_members, gz, member_offsets), "tokenize_fragments_file_gz", n_names, names,
                                     name_offsets, unk_id, out_n_barcodes, out_barcode_names, out_barcode_name_offsets,
                                     out_barcode_offsets, out_ids);
+} GT_CATCH
+
+extern "C" int32_t gtgpu_count_fragments_file(gtgpu_index* ix, const char* text, uint64_t n_bytes, uint32_t n_names, const char* names,
+                                              const uint32_t* name_offsets, uint32_t unk_id, uint32_t* out_n_barcodes,
+                                              gtgpu_buf** out_barcode_names, gtgpu_buf** out_barcode_name_offsets,
+                                              gtgpu_buf** out_barcode_offsets, gtgpu_buf** out_tokens, gtgpu_buf** out_counts) try {
+    return count_fragments_file(ix, TextIn::plain(text, n_bytes), "count_fragments_file", n_names, names, name_offsets, unk_id,
+                                out_n_barcodes, out_barcode_names, out_barcode_name_offsets, out_barcode_offsets, out_tokens, out_counts);
+} GT_CATCH
+
+extern "C" int32_t gtgpu_count_fragments_file_gz(gtgpu_index* ix, uint64_t n_members, const uint8_t* gz, const uint64_t* member_offsets,
+                                                 uint32_t n_names, const char* names, const uint32_t* name_offsets, uint32_t unk_id,
+                                                 uint32_t* out_n_barcodes, gtgpu_buf** out_barcode_names,
+                                                 gtgpu_buf** out_barcode_name_offsets, gtgpu_buf** out_barcode_offsets,
+                                                 gtgpu_buf** out_tokens, gtgpu_buf** out_counts) try {
+    return count_fragments_file(ix, TextIn::gzip(n_members, gz, member_offsets), "count_fragments_file_gz", n_names, names, name_offsets,
+                                unk_id, out_n_barcodes, out_barcode_names, out_barcode_name_offsets, out_barcode_offsets, out_tokens,
+                                out_counts);
 } GT_CATCH

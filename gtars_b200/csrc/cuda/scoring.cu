@@ -249,80 +249,89 @@ extern "C" int32_t gtgpu_score_matrix(gtgpu_index* ix, uint64_t n_files, const u
     return GTGPU_OK;
 } GT_CATCH
 
+int32_t gtgpu::reduce_pairs_csr_locked(gtgpu_ctx* ctx, uint64_t total, uint32_t* d_keys, uint32_t* d_vals, int val_bits, uint32_t n_keys,
+                                       uint64_t* out_key_offsets, gtgpu_buf** out_values, gtgpu_buf** out_counts, const std::string& who) {
+    cudaStream_t st = ctx->stream;
+    uint64_t nnz = 0;
+    uint32_t *d_val_out = nullptr, *d_count_out = nullptr;
+    if (total) {
+        uint32_t *d_k2, *d_v2;
+        unsigned long long *d_head, *d_rank, *d_runs;
+        void* d_tmp;
+        uint64_t* d_ko;
+        GT_TRY(ctx->scratch_get(SC_IN2_START, total * 4, (void**)&d_k2));
+        GT_TRY(ctx->scratch_get(SC_IN2_END, total * 4, (void**)&d_v2));
+        GT_TRY(ctx->scratch_get(SC_IN3_START, std::max(radix_sort_temp_bytes(total), exclusive_scan_temp_bytes(total, 8)), &d_tmp));
+        // stable LSD: by value first, then by key -> sorted by (key, value)
+        uint32_t *ka = d_vals, *va = d_keys, *kb = d_k2, *vb = d_v2;
+        int in_b = 0;
+        GT_TRY(radix_sort_pairs(ctx, total, ka, va, kb, vb, val_bits, d_tmp, &in_b));
+        if (in_b) { std::swap(ka, kb); std::swap(va, vb); }
+        // now (ka = values sorted, va = keys); second sort keys = keys, values = values
+        GT_TRY(radix_sort_pairs(ctx, total, va, ka, vb, kb, bits_for_value(n_keys ? n_keys - 1 : 0), d_tmp, &in_b));
+        uint32_t* s_key = in_b ? vb : va;
+        uint32_t* s_val = in_b ? kb : ka;
+        GT_TRY(ctx->scratch_get(SC_COUNTS, total * 8, (void**)&d_head));
+        GT_TRY(ctx->scratch_get(SC_IN3_CHR, total * 8, (void**)&d_rank));
+        GT_TRY(ctx->scratch_get(SC_IN3_END, total * 8, (void**)&d_runs));
+        const int g = grid_for(ctx, total);
+        score_run_heads_kernel<<<g, 256, 0, st>>>(total, s_key, s_val, d_head);
+        ctx->launches++;
+        GT_TRY(exclusive_scan<unsigned long long>(ctx, d_head, d_rank, total, d_tmp));
+        score_run_starts_kernel<<<g, 256, 0, st>>>(total, d_head, d_rank, d_runs);
+        ctx->launches++;
+        unsigned long long last[2];
+        GT_CUDA(cudaMemcpyAsync(&last[0], d_rank + total - 1, 8, cudaMemcpyDeviceToHost, st));
+        GT_CUDA(cudaMemcpyAsync(&last[1], d_head + total - 1, 8, cudaMemcpyDeviceToHost, st));
+        GT_CUDA(cudaStreamSynchronize(st));
+        nnz = last[0] + last[1];
+        GT_TRY(ctx->scratch_get(SC_OUT_IDS2, nnz * 8, (void**)&d_val_out));
+        d_count_out = d_val_out + nnz;
+        score_runs_out_kernel<<<grid_for(ctx, nnz), 256, 0, st>>>(nnz, total, d_runs, s_val, d_val_out, d_count_out);
+        GT_TRY(ctx->scratch_get(SC_FILE_TOK, ((uint64_t)n_keys + 1) * 8, (void**)&d_ko));
+        score_barcode_offsets_kernel<<<(n_keys + 1 + 255) / 256, 256, 0, st>>>(n_keys, nnz, d_runs, s_key, d_ko);
+        ctx->launches += 2;
+        GT_CUDA(cudaMemcpyAsync(out_key_offsets, d_ko, ((uint64_t)n_keys + 1) * 8, cudaMemcpyDeviceToHost, st));
+        GT_CUDA(cudaGetLastError());
+    }
+    if (nnz == 0)
+        for (uint32_t k = 0; k <= n_keys; ++k) out_key_offsets[k] = 0;
+
+    BufPtr values, counts;
+    int32_t s = buf_from_device(ctx, d_val_out, nnz, 4, st, &values);
+    if (s == GTGPU_OK) s = buf_from_device(ctx, d_count_out, nnz, 4, st, &counts);
+    if (s != GTGPU_OK) {
+        cudaStreamSynchronize(st);  // the values' copy may still run
+        return s == GTGPU_ERR_CUDA ? fail(s, who + ": D2H: " + gtgpu_last_error()) : s;
+    }
+    const cudaError_t e = cudaStreamSynchronize(st);
+    if (e != cudaSuccess) return fail(GTGPU_ERR_CUDA, who + ": " + cudaGetErrorString(e));
+    *out_values = values.release();
+    *out_counts = counts.release();
+    return GTGPU_OK;
+}
+
 // Device-resident core of gtgpu_score_barcodes (the caller holds ctx->mu): fragments and dense barcode ids on the device,
 // out_barcode_offsets (n_barcodes + 1) on the host.
 static int32_t score_barcodes_dev_locked(gtgpu_index* ix, uint64_t n, const uint32_t* d_chr, const uint32_t* d_start,
                                          const uint32_t* d_end, const uint32_t* d_bc, uint32_t n_barcodes,
                                          uint64_t* out_barcode_offsets, gtgpu_buf** out_peaks, gtgpu_buf** out_counts) {
     gtgpu_ctx* ctx = ix->ctx;
-    cudaStream_t st = ctx->stream;
-    uint64_t nnz = 0, total = 0;
-    uint32_t *d_peak_out = nullptr, *d_count_out = nullptr;
+    uint64_t total = 0;
+    uint32_t *d_ids = nullptr, *d_hbc = nullptr;
     if (n) {
         uint64_t* d_off;
         GT_TRY(ctx->scratch_get(SC_OUT_OFFS, (n + 1) * 8, (void**)&d_off));
-        uint32_t* d_ids = nullptr;
         GT_TRY(fused_find_all(ix, n, 0, nullptr, d_chr, d_start, d_end, d_off, nullptr, &d_ids, &total));
         if (total >= 0xFFFFFFFFull) return fail(GTGPU_ERR_UNSUPPORTED, "score_barcodes: more than 2^32-2 hits per call");
         if (total) {
-            uint32_t *d_hbc, *d_k2, *d_v2;
-            unsigned long long *d_head, *d_rank, *d_runs;
-            void* d_tmp;
-            uint64_t* d_bco;
             GT_TRY(ctx->scratch_get(SC_IN2_CHR, total * 4, (void**)&d_hbc));
-            GT_TRY(ctx->scratch_get(SC_IN2_START, total * 4, (void**)&d_k2));
-            GT_TRY(ctx->scratch_get(SC_IN2_END, total * 4, (void**)&d_v2));
-            GT_TRY(ctx->scratch_get(SC_IN3_START, std::max(radix_sort_temp_bytes(total), exclusive_scan_temp_bytes(total, 8)), &d_tmp));
-            score_hit_barcodes_kernel<<<grid_for(ctx, n), 256, 0, st>>>(n, d_off, d_bc, d_hbc);
+            score_hit_barcodes_kernel<<<grid_for(ctx, n), 256, 0, ctx->stream>>>(n, d_off, d_bc, d_hbc);
             ctx->launches++;
-            // stable LSD: by peak first, then by barcode -> sorted by (barcode, peak)
-            uint32_t *ka = d_ids, *va = d_hbc, *kb = d_k2, *vb = d_v2;
-            int in_b = 0;
-            GT_TRY(radix_sort_pairs(ctx, total, ka, va, kb, vb, bits_for_value(ix->max_val), d_tmp, &in_b));
-            if (in_b) { std::swap(ka, kb); std::swap(va, vb); }
-            // now (ka = peaks sorted, va = barcodes); second sort keys = barcodes, values = peaks
-            GT_TRY(radix_sort_pairs(ctx, total, va, ka, vb, kb, bits_for_value(n_barcodes ? n_barcodes - 1 : 0), d_tmp, &in_b));
-            uint32_t* s_bc = in_b ? vb : va;
-            uint32_t* s_pk = in_b ? kb : ka;
-            GT_TRY(ctx->scratch_get(SC_COUNTS, total * 8, (void**)&d_head));
-            GT_TRY(ctx->scratch_get(SC_IN3_CHR, total * 8, (void**)&d_rank));
-            GT_TRY(ctx->scratch_get(SC_IN3_END, total * 8, (void**)&d_runs));
-            const int g = grid_for(ctx, total);
-            score_run_heads_kernel<<<g, 256, 0, st>>>(total, s_bc, s_pk, d_head);
-            ctx->launches++;
-            GT_TRY(exclusive_scan<unsigned long long>(ctx, d_head, d_rank, total, d_tmp));
-            score_run_starts_kernel<<<g, 256, 0, st>>>(total, d_head, d_rank, d_runs);
-            ctx->launches++;
-            unsigned long long last[2];
-            GT_CUDA(cudaMemcpyAsync(&last[0], d_rank + total - 1, 8, cudaMemcpyDeviceToHost, st));
-            GT_CUDA(cudaMemcpyAsync(&last[1], d_head + total - 1, 8, cudaMemcpyDeviceToHost, st));
-            GT_CUDA(cudaStreamSynchronize(st));
-            nnz = last[0] + last[1];
-            GT_TRY(ctx->scratch_get(SC_OUT_IDS2, nnz * 8, (void**)&d_peak_out));
-            d_count_out = d_peak_out + nnz;
-            score_runs_out_kernel<<<grid_for(ctx, nnz), 256, 0, st>>>(nnz, total, d_runs, s_pk, d_peak_out, d_count_out);
-            GT_TRY(ctx->scratch_get(SC_FILE_TOK, ((uint64_t)n_barcodes + 1) * 8, (void**)&d_bco));
-            score_barcode_offsets_kernel<<<(n_barcodes + 1 + 255) / 256, 256, 0, st>>>(n_barcodes, nnz, d_runs, s_bc, d_bco);
-            ctx->launches += 2;
-            GT_CUDA(cudaMemcpyAsync(out_barcode_offsets, d_bco, ((uint64_t)n_barcodes + 1) * 8, cudaMemcpyDeviceToHost, st));
-            GT_CUDA(cudaGetLastError());
         }
     }
-    if (nnz == 0)
-        for (uint32_t b = 0; b <= n_barcodes; ++b) out_barcode_offsets[b] = 0;
-
-    BufPtr peaks, counts;
-    int32_t s = buf_from_device(ctx, d_peak_out, nnz, 4, st, &peaks);
-    if (s == GTGPU_OK) s = buf_from_device(ctx, d_count_out, nnz, 4, st, &counts);
-    if (s != GTGPU_OK) {
-        cudaStreamSynchronize(st);  // the peaks' copy may still run
-        return s == GTGPU_ERR_CUDA ? fail(s, std::string("score_barcodes: D2H: ") + gtgpu_last_error()) : s;
-    }
-    const cudaError_t e = cudaStreamSynchronize(st);
-    if (e != cudaSuccess) return fail(GTGPU_ERR_CUDA, std::string("score_barcodes: ") + cudaGetErrorString(e));
-    *out_peaks = peaks.release();
-    *out_counts = counts.release();
-    return GTGPU_OK;
+    return reduce_pairs_csr_locked(ctx, total, d_hbc, d_ids, bits_for_value(ix->max_val), n_barcodes, out_barcode_offsets, out_peaks,
+                                   out_counts, "score_barcodes");
 }
 
 extern "C" int32_t gtgpu_score_barcodes(gtgpu_index* ix, uint64_t n, const uint32_t* chr, const uint32_t* start,

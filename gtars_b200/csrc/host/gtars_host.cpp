@@ -993,6 +993,36 @@ std::vector<std::pair<std::string, std::map<uint32_t, uint32_t>>> Tokenizer::cou
     return out;
 }
 
+std::vector<std::pair<std::string, std::map<uint32_t, uint32_t>>> Tokenizer::count_fragments_by_barcode_device(const std::string& path) const {
+    NameBlob nb(cmap_);
+    uint32_t n_barcodes = 0;
+    PinnedResult names, name_offsets, offs, tokens, counts;
+    {
+        const FileBytes fb(path);
+        if (fb.gz)  // bgzip'ed fragment file: inflated and parsed on the device
+            check(gtgpu_count_fragments_file_gz(index_, fb.members.size() - 1, (const uint8_t*)fb.raw.data(), fb.members.data(),
+                                                (uint32_t)cmap_.size(), nb.blob.data(), nb.offsets.data(), unk_id_, &n_barcodes,
+                                                &names.buf, &name_offsets.buf, &offs.buf, &tokens.buf, &counts.buf),
+                  "gtgpu_count_fragments_file_gz");
+        else
+            check(gtgpu_count_fragments_file(index_, fb.text.data(), fb.text.size(), (uint32_t)cmap_.size(), nb.blob.data(),
+                                             nb.offsets.data(), unk_id_, &n_barcodes, &names.buf, &name_offsets.buf, &offs.buf,
+                                             &tokens.buf, &counts.buf),
+                  "gtgpu_count_fragments_file");
+    }
+    const char* blob = (const char*)gtgpu_buf_data(names.buf);
+    const uint64_t* noff = (const uint64_t*)gtgpu_buf_data(name_offsets.buf);
+    const uint64_t* off = (const uint64_t*)gtgpu_buf_data(offs.buf);
+    std::vector<std::pair<std::string, std::map<uint32_t, uint32_t>>> out;
+    out.reserve(n_barcodes);
+    for (uint32_t b = 0; b < n_barcodes; ++b) {
+        std::map<uint32_t, uint32_t> m;
+        for (uint64_t k = off[b]; k < off[b + 1]; ++k) m.emplace_hint(m.end(), tokens.data()[k], counts.data()[k]);
+        out.emplace_back(std::string(blob + noff[b], noff[b + 1] - noff[b]), std::move(m));
+    }
+    return out;
+}
+
 // ---- IndexedRegionSet ---------------------------------------------------------------------------------------------------------
 IndexedRegionSet::IndexedRegionSet(std::shared_ptr<Device> dev, RegionSet regions, OverlapperType kind)
     : source_(std::move(regions)), index_(new MultiChromOverlapper(std::move(dev), source_, kind)) {}

@@ -255,6 +255,9 @@ class Tokenizer {
     std::vector<std::pair<std::string, std::vector<uint32_t>>> tokenize_fragment_file_device(const std::string& path) const;
     // utils/fragments.rs:87-112: barcode -> (token id -> count).
     std::vector<std::pair<std::string, std::map<uint32_t, uint32_t>>> count_fragments_by_barcode(const std::string& path) const;
+    // The same with the file parsed, tokenized and counted on the device (gtgpu_count_fragments_file / _gz, bgzip'ed files inflated
+    // there too); barcodes in first-appearance order.
+    std::vector<std::pair<std::string, std::map<uint32_t, uint32_t>>> count_fragments_by_barcode_device(const std::string& path) const;
 
     size_t get_vocab_size() const { return universe_.len(); }
     int64_t convert_token_to_id(const std::string& tok) const;

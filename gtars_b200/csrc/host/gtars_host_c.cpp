@@ -29,6 +29,17 @@ std::vector<const RegionSet*> as_sets(uint64_t n, void** handles) {
     for (uint64_t i = 0; i < n; ++i) v[i] = (const RegionSet*)handles[i];
     return v;
 }
+
+Lists* count_lists(const std::vector<std::pair<std::string, std::map<uint32_t, uint32_t>>>& counts) {
+    Lists* l = new Lists();
+    for (auto& kv : counts) {
+        l->names.push_back(kv.first);
+        std::vector<uint32_t> flat;
+        for (auto& tc : kv.second) { flat.push_back(tc.first); flat.push_back(tc.second); }
+        l->lists.push_back(std::move(flat));
+    }
+    return l;
+}
 }  // namespace
 
 extern "C" {
@@ -311,6 +322,13 @@ void* gth_tokenizer_fragments(void* t, const char* path) {
         }
         return l;
     }, nullptr);
+}
+// barcode -> interleaved (token id, count) pairs
+void* gth_tokenizer_count_fragments(void* t, const char* path) {
+    return guard([&]() -> void* { return count_lists(((Tokenizer*)t)->count_fragments_by_barcode(path)); }, nullptr);
+}
+void* gth_tokenizer_count_fragments_device(void* t, const char* path) {
+    return guard([&]() -> void* { return count_lists(((Tokenizer*)t)->count_fragments_by_barcode_device(path)); }, nullptr);
 }
 
 // ---- Igd / LOLA -------------------------------------------------------------------------------------------------------------------

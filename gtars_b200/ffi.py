@@ -67,6 +67,8 @@ SIGNATURES = {
     "gtgpu_tokenize_fragments_gz": (_i32, [_vp, _u64, _vp, _vp, _u32, _vp, _vp, _u32, _vp, _vp, _vp, _vp, _vp]),
     "gtgpu_tokenize_fragments_file": (_i32, [_vp, _vp, _u64, _u32, _vp, _vp, _u32, _vp, _vp, _vp, _vp, _vp]),
     "gtgpu_tokenize_fragments_file_gz": (_i32, [_vp, _u64, _vp, _vp, _u32, _vp, _vp, _u32, _vp, _vp, _vp, _vp, _vp]),
+    "gtgpu_count_fragments_file": (_i32, [_vp, _vp, _u64, _u32, _vp, _vp, _u32, _vp, _vp, _vp, _vp, _vp, _vp]),
+    "gtgpu_count_fragments_file_gz": (_i32, [_vp, _u64, _vp, _vp, _u32, _vp, _vp, _u32, _vp, _vp, _vp, _vp, _vp, _vp]),
     "gtgpu_score_matrix": (_i32, [_vp, _u64, _vp, _u64, _vp, _vp, _vp, _i32, _u64, _vp]),
     "gtgpu_score_matrix_dev": (_i32, [_vp, _u64, _vp, _u64, _vp, _vp, _vp, _i32, _u64, _vp]),
     "gtgpu_score_barcodes": (_i32, [_vp, _u64, _vp, _vp, _vp, _vp, _u32, _vp, _vp, _vp]),
@@ -449,6 +451,24 @@ class Index:
         names = _take(hn, dtype=np.uint8).tobytes()
         no = _take(hno, dtype=np.uint64)
         return [names[int(a):int(b)].decode() for a, b in zip(no[:-1], no[1:])], _take(ho, dtype=np.uint64), _take(hi)
+
+    def count_fragments_file(self, text, chrom_names, unk_id, gz_member_offsets=None):
+        """gtgpu_count_fragments_file (or _gz when gz_member_offsets is given: `text` is then the gzip data), any size:
+        ([barcode strings], offsets[n + 1], tokens, counts); per barcode its distinct token ids ascending, with their counts."""
+        blob, offs = _names_blob(chrom_names)
+        nb = C.c_uint32(0)
+        hn, hno, ho, ht, hc = C.c_void_p(), C.c_void_p(), C.c_void_p(), C.c_void_p(), C.c_void_p()
+        outs = (C.byref(nb), C.byref(hn), C.byref(hno), C.byref(ho), C.byref(ht), C.byref(hc))
+        if gz_member_offsets is not None:
+            mo = _arr(gz_member_offsets, np.uint64)
+            check(lib().gtgpu_count_fragments_file_gz(self._h, len(mo) - 1, _text_ptr(text), _p(mo), len(chrom_names), blob, _p(offs),
+                                                      unk_id, *outs))
+        else:
+            check(lib().gtgpu_count_fragments_file(self._h, _text_ptr(text), _text_len(text), len(chrom_names), blob, _p(offs), unk_id,
+                                                   *outs))
+        names = _take(hn, dtype=np.uint8).tobytes()
+        no = _take(hno, dtype=np.uint64)
+        return ([names[int(a):int(b)].decode() for a, b in zip(no[:-1], no[1:])], _take(ho, dtype=np.uint64), _take(ht), _take(hc))
 
     def score_matrix(self, file_offsets, chr, start, end, mode, n_cols):
         """region_scoring_from_fragments: uint32 [n_files, n_cols]."""

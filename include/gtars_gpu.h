@@ -336,6 +336,22 @@ int32_t gtgpu_tokenize_fragments_file_gz(gtgpu_index* index, uint64_t n_members,
                                          uint32_t* out_n_barcodes, gtgpu_buf** out_barcode_names, gtgpu_buf** out_barcode_name_offsets,
                                          gtgpu_buf** out_barcode_offsets, gtgpu_buf** out_ids);
 
+/* count_fragments_by_barcode (gtars-tokenizers/src/utils/fragments.rs:87-112) from ONE fragment file's bytes of any size, parsed on
+ * the device: the cell x token count table of the ids gtgpu_tokenize_fragments_file returns.  Input forms, line rules, errors
+ * ("Invalid fragment file detected at line: i", no output), windows and limits are those of gtgpu_tokenize_fragments_file, and so
+ * are *out_n_barcodes, *out_barcode_names and *out_barcode_name_offsets (every barcode, first-appearance order).
+ * *out_barcode_offsets = n_barcodes + 1 u64 offsets into *out_tokens / *out_counts (u32 each): per barcode its distinct token ids
+ * in ascending order and how often each occurs.  A fragment with no hit, or on an unknown chromosome, counts once under unk_id,
+ * so every barcode has at least one entry.  On a multi-device ctx these run on the first device. */
+int32_t gtgpu_count_fragments_file(gtgpu_index* index, const char* text, uint64_t n_bytes, uint32_t n_names, const char* names,
+                                   const uint32_t* name_offsets, uint32_t unk_id, uint32_t* out_n_barcodes,
+                                   gtgpu_buf** out_barcode_names, gtgpu_buf** out_barcode_name_offsets,
+                                   gtgpu_buf** out_barcode_offsets, gtgpu_buf** out_tokens, gtgpu_buf** out_counts);
+int32_t gtgpu_count_fragments_file_gz(gtgpu_index* index, uint64_t n_members, const uint8_t* gz, const uint64_t* member_offsets,
+                                      uint32_t n_names, const char* names, const uint32_t* name_offsets, uint32_t unk_id,
+                                      uint32_t* out_n_barcodes, gtgpu_buf** out_barcode_names, gtgpu_buf** out_barcode_name_offsets,
+                                      gtgpu_buf** out_barcode_offsets, gtgpu_buf** out_tokens, gtgpu_buf** out_counts);
+
 /* ---- gtars-scoring: fragments x consensus peaks ------------------------------------------------------------------------
  * gtgpu_score_matrix replaces region_scoring_from_fragments (gtars-scoring/src/fragment_scoring.rs:19-121) over
  * pre-parsed fragments: file f owns fragments [file_offsets[f], file_offsets[f+1]); the index is the ConsensusSet
